@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repository's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference's own C++ on the host cores (oracle/_ref)
+    python bench.py ... --dump-outputs DIR                   # also write each config's last timed outputs to DIR/*.npy
 
 A "step" is one whole scde.expression.difference over one synthetic count matrix: device dedup of the counts,
 log-posterior table, the bootstrap joint posteriors of both groups, the sliding-product ratio posterior and the
@@ -64,7 +65,14 @@ def parse_args():
                     help="scde_b200_options field (e.g. item_order=1, hot_rank=16); repeatable")
     ap.add_argument("--trace", action="store_true", help="host wall-clock of the one-shot call's phases on stderr")
     ap.add_argument("--boot", type=int, default=None, help="n.randomizations (default 100, BASELINE.json; R's default is 150)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step of each config returned (grid indices, "
+                         "Z, BH-corrected cZ) as DIR/cfg<N>_<name>.npy in float64")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
     if args.boot:
         global N_BOOT
         N_BOOT = args.boot
@@ -330,6 +338,7 @@ class Bench:
             self.ctx.set_options(**opts)
         self.opts = opts
         self.ext = torch.cuda.ExternalStream(self.ctx.stream, device=self.device)
+        self.outputs = {}  # rank 0: "cfg<N>" -> what the last timed step of that config returned
 
     def barrier(self):
         if self.world > 1:
@@ -445,6 +454,8 @@ class Bench:
         ms_step, stats_acc, full = timed_resident(job, G_all, steps, max(0, warmup - 1))
         clocks = sampler.stop()
         job.close()
+        if rank == 0:
+            self.outputs[f"cfg{config}"] = full
 
         # ---------------- end-to-end arm: host buffers through the one-shot C-ABI call ----------------
         n_draw_sets = 4 if batch is not None else 2
@@ -461,7 +472,7 @@ class Bench:
 
         e2e_step((g0, g1), G_all)
         self.barrier()
-        e2e_steps = max(1, min(steps, 5))
+        e2e_steps = steps
         e2, e3 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         with torch.cuda.stream(ext):
             e2.record(ext)  # the stream is idle here, so this timestamps the start of the host call
@@ -475,7 +486,7 @@ class Bench:
         weak = None
         if world > 1 and sharded and not self.args.no_weak:
             wjob = make_job((0, G_all))
-            wms, _, _ = timed_resident_local(self, wjob, min(steps, 3), 1)
+            wms, _, _ = timed_resident_local(self, wjob, steps, 1)
             wjob.close()
             weak = wms
 
@@ -648,6 +659,24 @@ def timed_resident_local(b: Bench, job, n_steps, n_warm):
     return e0.elapsed_time(e1) / n_steps, None, None
 
 
+def dump_outputs(outputs, out_dir, max_bytes=60_000_000):
+    """Writes every array of `outputs` ({"cfg<N>": {name: array}}) as out_dir/cfg<N>_<name>.npy in float64 (grid indices
+    are small integers, exact in float64).  Where all of it would exceed max_bytes, every config keeps the same fixed,
+    seeded sample of gene rows in each of its arrays, and the sampled rows are written as cfg<N>_genes.npy."""
+    row_bytes = {cfg: 8 + sum(8 * np.asarray(v)[0].size for v in res.values()) for cfg, res in outputs.items()}
+    total = sum(len(res["z"]) * row_bytes[cfg] for cfg, res in outputs.items())
+    keep = min(1.0, max_bytes / max(1, total))
+    os.makedirs(out_dir, exist_ok=True)
+    for cfg, res in outputs.items():
+        n_genes = len(res["z"])
+        rows = slice(None)
+        if keep < 1.0:
+            rows = np.sort(np.random.default_rng(0).choice(n_genes, int(n_genes * keep), replace=False))
+            np.save(os.path.join(out_dir, f"{cfg}_genes.npy"), rows.astype(np.float64))
+        for name, v in res.items():
+            np.save(os.path.join(out_dir, f"{cfg}_{name}.npy"), np.ascontiguousarray(np.asarray(v)[rows], dtype=np.float64))
+
+
 def main():
     args = parse_args()
     rank = int(os.environ.get("RANK", "0"))
@@ -663,7 +692,7 @@ def main():
         subs = {}
         for cfg in (3, 5):
             g, c = config_size(cfg)
-            sub = b.measure(cfg, g, c, max(2, min(args.steps, 5)), 2, with_cpu=not args.no_cpu_baseline,
+            sub = b.measure(cfg, g, c, args.steps, 2, with_cpu=not args.no_cpu_baseline,
                             with_parity=not args.no_parity, sample_per_core=2 if cfg == 5 else 8)
             if sub is not None:
                 keep = ("value", "unit", "n_gpus", "ms_per_step", "scaling", "config", "e2e", "parity", "shard_parity",
@@ -673,6 +702,8 @@ def main():
                 subs[f"cfg{cfg}"]["stage_ms"] = sub["roofline"]["stage_ms"]
         if line is not None:
             line["sub_records"] = subs
+    if args.dump_outputs and b.rank == 0:
+        dump_outputs(b.outputs, args.dump_outputs)
     if line is not None:
         print(json.dumps(line), flush=True)
     if world > 1:

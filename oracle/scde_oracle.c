@@ -12,8 +12,9 @@
  * oracle/shim/RcppArmadillo.h (the part of R / Rcpp / Armadillo they use, restated; Makefile target
  * `ref` -> oracle/_ref/libscde_ref.so).  tests/test_ref.py holds every entry point of this file to
  * that library BIT FOR BIT (all returnpost forms, batch, ensemble, no-bootstrap, local theta, legacy
- * forms, matSlideMult, the rand() rejection loop), and tests/golden/ref_fixtures.npz carries its
- * outputs to machines without /root/reference.  What stays restated -- "parity unpinned" in the
+ * forms, matSlideMult, the rand() rejection loop; without the library, against the digests of its
+ * outputs in tests/golden/ref_digests.json), and tests/golden/ref_fixtures_*.npz keeps outputs of
+ * it.  What stays restated -- "parity unpinned" in the
  * strict sense -- is R itself: nmath's dnbinom / dpois (used by BOTH sides through Rf_dnbinom /
  * Rf_dpois of the shim), qnorm / pnorm / p.adjust and the R-level ratio-posterior / summary code
  * (R/functions.R), pinned by (a) mpmath 50-digit values, (b) scipy ndtri, (c) numpy.correlate,

@@ -1,6 +1,6 @@
-"""Writes tests/golden/ref_fixtures.npz: outputs of THE REFERENCE'S OWN C++ (src/jpmatLogBoot.cpp, src/matSlideMult.cpp
-compiled unmodified against oracle/shim -> oracle/_ref/libscde_ref.so) on committed inputs.  Run in the authoring
-container only (/root/reference does not exist on the GPU box); the fixtures travel.
+"""Writes tests/golden/ref_fixtures_*.npz: outputs of THE REFERENCE'S OWN C++ (src/jpmatLogBoot.cpp, src/matSlideMult.cpp
+compiled unmodified against oracle/shim -> oracle/_ref/libscde_ref.so) on committed inputs.  Runs only where the
+reference's sources are present (SCDE_REF_SRC); the tests use the committed fixtures.
 
     python tests/golden/make_ref_fixtures.py
 
@@ -65,9 +65,11 @@ def main():
     flat, off, uci = O.unique_counts(counts)
     r = R.log_boot_posterior(mm, flat, off, uci, mag, 50, seed=1, returnpost=1, localtheta=lt, sqlogit=sq)
     out["knn_jp"], out["knn_modes"] = r["jp"], r["modes"]
-    path = os.path.join(HERE, "ref_fixtures.npz")
-    np.savez_compressed(path, **out)
-    print(path, os.path.getsize(path), {k: v.shape for k, v in out.items()})
+    for name, prefix in helpers.REF_FIXTURE_FILES.items():
+        path = os.path.join(HERE, name)
+        part = {k: v for k, v in out.items() if k.startswith(prefix)}
+        np.savez_compressed(path, **part)
+        print(path, os.path.getsize(path), {k: v.shape for k, v in part.items()})
 
 
 if __name__ == "__main__":

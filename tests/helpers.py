@@ -57,12 +57,21 @@ def es_mef_inputs(variant: str = "tests"):
     return cd, ifm, prior, groups
 
 
-# ---- inputs of tests/golden/ref_fixtures.npz (outputs of the reference's own C++, tests/golden/make_ref_fixtures.py) ----
+# ---- inputs of tests/golden/ref_fixtures_*.npz (outputs of the reference's own C++, tests/golden/make_ref_fixtures.py) ----
 VIGNETTE_GENES = ["Dppa5a", "Pou5f1", "Gm13242", "Tdh", "Ift46", "4930509G22Rik"]
 
 
+REF_FIXTURE_FILES = {"ref_fixtures_cfg1.npz": "cfg1_", "ref_fixtures_batch_knn.npz": ("batch_", "knn_")}
+
+
+@functools.lru_cache(maxsize=None)
 def ref_fixtures():
-    return np.load(os.path.join(GOLD, "ref_fixtures.npz"))
+    """{name: array} of both fixture files (split by case so that each stays under 1 MB)"""
+    out = {}
+    for name in REF_FIXTURE_FILES:
+        with np.load(os.path.join(GOLD, name)) as d:
+            out.update({k: d[k] for k in d.files})
+    return out
 
 
 def ref_cfg1_inputs():

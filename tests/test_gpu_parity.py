@@ -704,7 +704,7 @@ def test_second_device_runs_every_kernel(ctx):
 
 
 def test_cuda_path_against_reference_fixtures(ctx):
-    """The CUDA path against outputs of THE REFERENCE'S OWN C++ (tests/golden/ref_fixtures.npz: src/jpmatLogBoot.cpp and
+    """The CUDA path against outputs of THE REFERENCE'S OWN C++ (tests/golden/ref_fixtures_*.npz: src/jpmatLogBoot.cpp and
     src/matSlideMult.cpp compiled unmodified, tests/golden/make_ref_fixtures.py) -- no oracle in between.  Config 1's
     data incl. the vignette's six genes, a batch case, the 12-column knn models.  Log-posteriors 1e-6 relative, modes
     exact, matSlideMult bit-exact."""
@@ -826,7 +826,7 @@ def test_r_shim_symbols_against_reference_fixtures(ctx):
 
     path = os.path.join(helpers.GOLD, "..", "..", "integration", "_build", "libscde_shim.so")
     if not os.path.exists(path):
-        pytest.skip("integration/_build/libscde_shim.so not built (make -C integration; needs the reference headers)")
+        pytest.fail("integration/_build/libscde_shim.so is missing: __graft_entry__.build() builds it (make -C integration)")
     shim = ctypes.CDLL(os.path.abspath(path))
     keep, R._lib = R._lib, shim  # the oracle.ref binding, pointed at the shim build of the same five entry points
     try:
@@ -935,7 +935,7 @@ def test_r_shim_fused_entry(ctx, batch):
 
     path = os.path.abspath(os.path.join(helpers.GOLD, "..", "..", "integration", "_build", "libscde_shim.so"))
     if not os.path.exists(path):
-        pytest.skip("integration/_build/libscde_shim.so not built")
+        pytest.fail("integration/_build/libscde_shim.so is missing: __graft_entry__.build() builds it (make -C integration)")
     shim = ctypes.CDLL(path)
     w = synth.make_workload(5 if batch else 3, n_genes=120, n_cells=40, seed=29, batch=batch)
     mm, lt, sq = api.pack_models(w.models)

@@ -122,14 +122,6 @@ def test_argument_validation_mirrors_reference():
         api.scde_posteriors(w.models, w.counts, w.prior, batch=pd.Categorical(list("ababab")))
 
 
-def test_rdata_reader_matches_fixtures():
-    if not os.path.exists("/root/reference/data/o.ifm.rda"):
-        pytest.skip("reference data not present on this box")
-    from scde_b200.rdata import as_data_frame, read_rda
-    ifm = as_data_frame(read_rda("/root/reference/data/o.ifm.rda")["o.ifm"])
-    assert np.array_equal(ifm.to_numpy(), helpers.o_ifm().to_numpy()) and list(ifm.index) == list(helpers.o_ifm().index)
-
-
 def test_expression_prior_shapes_match_survey_probes():
     cd, ifm, prior, groups = helpers.es_mef_inputs("tests")
     assert cd.shape == (13788, 40) and len(prior) == 401 and prior["x"].iloc[0] == 0.0

@@ -167,10 +167,10 @@ def test_oracle_reproduces_committed_golden_slice():
 
 
 def test_oracle_matches_reference_fixtures():
-    """tests/golden/ref_fixtures.npz holds outputs of the reference's own C++ (src/jpmatLogBoot.cpp, src/matSlideMult.cpp
+    """tests/golden/ref_fixtures_*.npz holds outputs of the reference's own C++ (src/jpmatLogBoot.cpp, src/matSlideMult.cpp
     compiled unmodified, tests/golden/make_ref_fixtures.py).  The oracle reproduces them BIT FOR BIT on config 1's data
     (es.mef.small + o.ifm, incl. the vignette's six genes), a batch case and the 12-column knn models -- this is what
-    pins the oracle where /root/reference (and oracle/_ref) is absent."""
+    pins the oracle without the reference's sources (which the repository does not carry)."""
     fx = helpers.ref_fixtures()
     sub, ifm, prior, groups, sel = helpers.ref_cfg1_inputs()
     assert np.array_equal(sel, fx["cfg1_genes"])
