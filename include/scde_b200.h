@@ -282,6 +282,75 @@ SCDE_B200_API int scde_b200_diff_download(scde_b200_ctx *ctx, scde_b200_diff_job
                             scde_b200_stats *stats);
 SCDE_B200_API void scde_b200_diff_free(scde_b200_ctx *ctx, scde_b200_diff_job *job);
 
+/* ---- many contrasts on one resident dataset ------------------------------------------------- */
+/*
+ * A dataset holds the count matrix, its unique-count index and the log-posterior table of ALL its cells on the device, so
+ * that any number of two-group contrasts over those cells can be computed without rebuilding them.  Every contrast (A, B)
+ * returns bit for bit what scde_b200_expression_difference returns for the same data, options, n_boot, seed, expectation
+ * and batch, with group code 0 on A's cells, 1 on B's cells and -1 on every other cell -- except where the tcgen05
+ * contraction had to fall back to the FP64 kernel (see DESIGN.md, "Many contrasts"): there the affected contrasts agree
+ * with the one-shot call within the oracle tolerances.
+ *
+ * Each group's joint posterior is computed once per call however many contrasts name it (the draws of a group depend on
+ * the seed, n_boot and the group's size only), and each distinct batch composition's joint once.
+ *
+ * A dataset holds its context's differential-expression workspace until scde_b200_dataset_free: while it is alive,
+ * scde_b200_expression_difference, scde_b200_diff_upload and a second scde_b200_dataset_create on that context fail with
+ * SCDE_B200_EINVAL ("another expression_difference job is alive").  On a scde_b200_create_multi context the dataset is one
+ * per-device dataset per contiguous gene range (the split of scde_b200_expression_difference).
+ */
+typedef struct {
+    int32_t n_genes, n_cells, n_grid;
+    const int32_t *counts;   /* n_genes x n_cells raw counts, cells ordered as the model rows */
+    const double *models;    /* n_cells x 12 (corr.a already clamped to >= 1e-10 by the caller) */
+    const double *prior_x;   /* n_grid */
+    const double *prior_y;   /* n_grid */
+    int32_t local_theta, square_logit_conc;
+} scde_b200_dataset_args;
+
+typedef struct {
+    /* groups as flattened cell lists: group i = group_cells[group_offsets[i] .. group_offsets[i+1]), model-row ids in
+     * ascending order, at least one cell each.  Groups may share cells, except the two groups of one contrast. */
+    int32_t n_groups;
+    const int32_t *group_offsets;  /* n_groups + 1 */
+    const int32_t *group_cells;
+    int32_t n_contrasts;
+    const int32_t *pairs;          /* 2 * n_contrasts group ids: contrast c is (pairs[2c], pairs[2c+1]) = (A, B) */
+    int32_t n_boot, seed;
+    const int32_t *zero_index;     /* as in scde_b200_diff_args, shared by every contrast */
+    int32_t n_zero;
+    const int32_t *zero_index_adjusted;
+    const int32_t *batch;          /* n_cells batch level codes (< 0 = NA) or NULL */
+    int32_t n_batch_levels;
+    const double *batch_models;    /* n_cells x 12 or NULL (= models), with their own column-presence flags */
+    int32_t batch_local_theta, batch_square_logit_conc;
+} scde_b200_contrast_args;
+
+/* Outputs, any pointer may be NULL.  Per-contrast blocks back to back: contrast c's block of a G x m output starts at
+ * c * G * m (G = the dataset's genes) and is column-major like the matching scde_b200_diff_out field.  cz, batch_cz and
+ * adjusted_cz are Benjamini-Hochberg over all genes of the contrast and need the matching z output. */
+typedef struct {
+    int32_t *idx;            /* n_contrasts x (G x 3) */
+    double *z, *cz;          /* n_contrasts x G */
+    int32_t *batch_idx;
+    double *batch_z, *batch_cz;
+    int32_t *adjusted_idx;
+    double *adjusted_z, *adjusted_cz;
+    double *difference_posterior;          /* n_contrasts x (G x (2K-1)) */
+    double *adjusted_difference_posterior; /* n_contrasts x (G x (4K-3)), batch only */
+    double *joint_posteriors;              /* n_groups x (G x K); groups that no contrast names are left untouched */
+} scde_b200_contrast_out;
+
+typedef struct scde_b200_dataset scde_b200_dataset;
+/* uploads the counts, builds the index and the table; stats (may be NULL) report the dedup and table stages */
+SCDE_B200_API int scde_b200_dataset_create(scde_b200_ctx *ctx, const scde_b200_dataset_args *args, scde_b200_dataset **out,
+                                           scde_b200_stats *stats);
+/* every contrast of `args` in one call; stats (may be NULL): launches[CONTRACT] and contract_cells count one contraction
+ * per distinct group and one per pair of batch joints */
+SCDE_B200_API int scde_b200_dataset_contrasts(scde_b200_ctx *ctx, scde_b200_dataset *ds, const scde_b200_contrast_args *args,
+                                              const scde_b200_contrast_out *out, scde_b200_stats *stats);
+SCDE_B200_API void scde_b200_dataset_free(scde_b200_ctx *ctx, scde_b200_dataset *ds);
+
 /* scde.expression.magnitude: out[g + G*c] = (log(counts[g + G*c]) - corr_b[c]) / corr_a[c] */
 SCDE_B200_API int scde_b200_expression_magnitude(scde_b200_ctx *ctx, const int32_t *counts, int32_t n_genes, int32_t n_cells,
                                    const double *corr_b, const double *corr_a, double *out);

@@ -251,3 +251,88 @@ RcppExport SEXP scde_b200_diff(SEXP Counts, SEXP Models, SEXP BatchModels, SEXP 
     out[8] = acz;
     return out;
 }
+
+// Many contrasts over one set of cells (scde_b200_dataset_*): the count matrix, its index and table are built once, each
+// group's joint posterior once, and every contrast is what scde_b200_diff returns for the two groups (codes 0 / 1, every
+// other cell NA).  Called by scde.expression.difference.contrasts.b200 (integration/scde_b200.R).
+//   GroupOffsets / GroupCells  the groups as 0-based ascending cell lists, flattened (length n.groups + 1 / total)
+//   Pairs                      2 x n.contrasts 0-based group ids, column c = (A, B) of contrast c
+//   BatchModels                cells x 12 or a 0 x 0 matrix (= Models), with its own BatchLocalThetaFit / BatchSquareLogitConc
+//                              flags (from colnames(batch.models))
+// Returns list(idx, z, cz[, batch.idx, batch.z, batch.cz, adjusted.idx, adjusted.z, adjusted.cz]): idx genes x (3 x
+// n.contrasts), contrast c in columns 3c+1 .. 3c+3 (lb, mle, ub, 0-based grid indices); z and cz genes x n.contrasts.
+RcppExport SEXP scde_b200_diff_contrasts(SEXP Counts, SEXP Models, SEXP BatchModels, SEXP PriorX, SEXP PriorY,
+                                         SEXP GroupOffsets, SEXP GroupCells, SEXP Pairs, SEXP Batch, SEXP NBatchLevels,
+                                         SEXP Nboot, SEXP Seed, SEXP ZeroIndex, SEXP ZeroIndexAdjusted, SEXP LocalThetaFit,
+                                         SEXP SquareLogitConc, SEXP BatchLocalThetaFit, SEXP BatchSquareLogitConc,
+                                         SEXP Devices) {
+    Rcpp::IntegerMatrix counts(Counts);
+    Rcpp::NumericMatrix models(Models), bmodels(BatchModels);
+    Rcpp::NumericVector px(PriorX), py(PriorY);
+    Rcpp::IntegerVector goff(GroupOffsets), gcells(GroupCells), pairs(Pairs), batch(Batch), zi(ZeroIndex),
+        zia(ZeroIndexAdjusted), devs(Devices);
+    const int G = counts.nrow(), C = counts.ncol(), K = px.size(), nc = pairs.size() / 2;
+    const bool has_batch = batch.size() == C && Rcpp::as<int>(NBatchLevels) > 1;
+    scde_b200_dataset_args d = scde_b200_dataset_args();
+    d.n_genes = G;
+    d.n_cells = C;
+    d.n_grid = K;
+    d.counts = counts.begin();
+    d.models = models.begin();
+    d.prior_x = px.begin();
+    d.prior_y = py.begin();
+    d.local_theta = Rcpp::as<int>(LocalThetaFit);
+    d.square_logit_conc = Rcpp::as<int>(SquareLogitConc);
+    scde_b200_contrast_args a = scde_b200_contrast_args();
+    a.n_groups = goff.size() - 1;
+    a.group_offsets = goff.begin();
+    a.group_cells = gcells.begin();
+    a.n_contrasts = nc;
+    a.pairs = pairs.begin();
+    a.n_boot = Rcpp::as<int>(Nboot);
+    a.seed = Rcpp::as<int>(Seed);
+    a.zero_index = zi.begin();
+    a.n_zero = zi.size();
+    a.zero_index_adjusted = zia.begin();
+    a.batch = has_batch ? batch.begin() : NULL;
+    a.n_batch_levels = has_batch ? Rcpp::as<int>(NBatchLevels) : 0;
+    a.batch_models = (has_batch && bmodels.size() == C * 12) ? bmodels.begin() : NULL;
+    a.batch_local_theta = Rcpp::as<int>(BatchLocalThetaFit);
+    a.batch_square_logit_conc = Rcpp::as<int>(BatchSquareLogitConc);
+    const int n_sets = has_batch ? 3 : 1;
+    std::vector<int> idx((size_t)n_sets * 3 * G * nc);
+    std::vector<Rcpp::NumericMatrix> z, cz;
+    for (int s = 0; s < n_sets; ++s) {
+        z.push_back(Rcpp::NumericMatrix(G, nc));
+        cz.push_back(Rcpp::NumericMatrix(G, nc));
+    }
+    scde_b200_contrast_out o = scde_b200_contrast_out();
+    o.idx = idx.data();
+    o.z = z[0].begin();
+    o.cz = cz[0].begin();
+    if (has_batch) {
+        o.batch_idx = idx.data() + (size_t)3 * G * nc;
+        o.batch_z = z[1].begin();
+        o.batch_cz = cz[1].begin();
+        o.adjusted_idx = idx.data() + (size_t)6 * G * nc;
+        o.adjusted_z = z[2].begin();
+        o.adjusted_cz = cz[2].begin();
+    }
+    std::vector<int> dv(devs.begin(), devs.end());
+    scde_b200_ctx *ctx = context(dv);
+    scde_b200_dataset *ds = NULL;
+    check(scde_b200_dataset_create(ctx, &d, &ds, NULL));
+    const int rc = scde_b200_dataset_contrasts(ctx, ds, &a, &o, NULL);
+    const std::string msg = rc == SCDE_B200_OK ? std::string() : scde_b200_last_error();
+    scde_b200_dataset_free(ctx, ds);  // before any R error: the context must accept the next call
+    if (rc != SCDE_B200_OK) Rcpp::stop(msg);
+    Rcpp::List out(3 * n_sets);  // named by the R wrapper
+    for (int s = 0; s < n_sets; ++s) {
+        Rcpp::NumericMatrix m(G, 3 * nc);
+        for (size_t i = 0; i < (size_t)3 * G * nc; ++i) m.begin()[i] = idx[(size_t)s * 3 * G * nc + i];
+        out[3 * s] = m;
+        out[3 * s + 1] = z[s];
+        out[3 * s + 2] = cz[s];
+    }
+    return out;
+}

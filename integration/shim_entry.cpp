@@ -1,5 +1,5 @@
 // shim_entry.cpp -- test wrapper (not part of what goes into the R package): builds the .Call arguments of
-// scde_b200_diff (integration/scde_b200_shim.cpp) from plain arrays, calls it as R would, copies the result out.
+// scde_b200_diff and scde_b200_diff_contrasts (integration/scde_b200_shim.cpp) from plain arrays, calls it as R would, copies the result out.
 // Linked into integration/_build/libscde_shim.so only (tests/test_gpu_parity.py).
 #include <Rcpp.h>
 
@@ -8,6 +8,11 @@
 RcppExport SEXP scde_b200_diff(SEXP Counts, SEXP Models, SEXP BatchModels, SEXP PriorX, SEXP PriorY, SEXP Group, SEXP Batch,
                                SEXP NBatchLevels, SEXP Nboot, SEXP Seed, SEXP ZeroIndex, SEXP ZeroIndexAdjusted,
                                SEXP LocalThetaFit, SEXP SquareLogitConc, SEXP Devices);
+RcppExport SEXP scde_b200_diff_contrasts(SEXP Counts, SEXP Models, SEXP BatchModels, SEXP PriorX, SEXP PriorY,
+                                         SEXP GroupOffsets, SEXP GroupCells, SEXP Pairs, SEXP Batch, SEXP NBatchLevels,
+                                         SEXP Nboot, SEXP Seed, SEXP ZeroIndex, SEXP ZeroIndexAdjusted, SEXP LocalThetaFit,
+                                         SEXP SquareLogitConc, SEXP BatchLocalThetaFit, SEXP BatchSquareLogitConc,
+                                         SEXP Devices);
 
 namespace {
 SEXP ivec(const int *p, size_t n) {
@@ -46,6 +51,46 @@ extern "C" int shim_diff(const int *counts, int G, int C, const double *models12
             std::memcpy(out_idx + (size_t)s * 3 * G, r->list[3 * s]->dval.data(), sizeof(double) * 3 * G);
             std::memcpy(out_z + (size_t)s * G, r->list[3 * s + 1]->dval.data(), sizeof(double) * G);
             std::memcpy(out_cz + (size_t)s * G, r->list[3 * s + 2]->dval.data(), sizeof(double) * G);
+        }
+    } catch (const std::exception &e) {
+        std::strncpy(err, e.what(), 255);
+        err[255] = 0;
+        rc = -1;
+    }
+    ShimArena::get().clear();
+    return rc;
+}
+
+// scde_b200_diff_contrasts: groups as flattened 0-based cell lists, pairs[2 * n_contrasts]; batch models = models.
+// out_idx[n_sets * n_contrasts * 3 * G] (as doubles), out_z / out_cz[n_sets * n_contrasts * G], n_sets = 3 with a batch
+// factor (results, batch.effect, batch.adjusted), else 1; contrast c's block inside a set as in scde_b200_contrast_out.
+extern "C" int shim_diff_contrasts(const int *counts, int G, int C, const double *models12, const double *px, const double *py,
+                                   int K, const int *group_offsets, int n_groups, const int *group_cells, const int *pairs,
+                                   int n_contrasts, const int *batch, int n_levels, int nboot, int zero_index,
+                                   int zero_index_adj, const int *devices, int n_devices, double *out_idx, double *out_z,
+                                   double *out_cz, char *err) {
+    int rc = 0;
+    try {
+        SEXP cnt = ivec(counts, (size_t)G * C);
+        cnt->nrow = G;
+        cnt->ncol = C;
+        SEXP mm = dvec(models12, (size_t)C * 12);
+        mm->nrow = C;
+        mm->ncol = 12;
+        SEXP bm = dvec(models12, 0);
+        bm->nrow = bm->ncol = 0;
+        int one = 1, zero = 0;
+        SEXP r = scde_b200_diff_contrasts(cnt, mm, bm, dvec(px, K), dvec(py, K), ivec(group_offsets, n_groups + 1),
+                                          ivec(group_cells, group_offsets[n_groups]), ivec(pairs, 2 * (size_t)n_contrasts),
+                                          ivec(batch, batch ? C : 0), ivec(&n_levels, 1), ivec(&nboot, 1), ivec(&one, 1),
+                                          ivec(&zero_index, 1), ivec(&zero_index_adj, 1), ivec(&zero, 1), ivec(&zero, 1),
+                                          ivec(&zero, 1), ivec(&zero, 1), ivec(devices, n_devices));
+        const int n_sets = (int)r->list.size() / 3;
+        const size_t n3 = (size_t)3 * G * n_contrasts, n1 = (size_t)G * n_contrasts;
+        for (int s = 0; s < n_sets; ++s) {
+            std::memcpy(out_idx + s * n3, r->list[3 * s]->dval.data(), sizeof(double) * n3);
+            std::memcpy(out_z + s * n1, r->list[3 * s + 1]->dval.data(), sizeof(double) * n1);
+            std::memcpy(out_cz + s * n1, r->list[3 * s + 2]->dval.data(), sizeof(double) * n1);
         }
     } catch (const std::exception &e) {
         std::strncpy(err, e.what(), 255);

@@ -51,6 +51,37 @@ class DiffOut(C.Structure):
     ]
 
 
+class DatasetArgs(C.Structure):
+    """scde_b200_dataset_args (include/scde_b200.h)."""
+    _fields_ = [
+        ("n_genes", C.c_int32), ("n_cells", C.c_int32), ("n_grid", C.c_int32),
+        ("counts", i32p), ("models", f64p), ("prior_x", f64p), ("prior_y", f64p),
+        ("local_theta", C.c_int32), ("square_logit_conc", C.c_int32),
+    ]
+
+
+class ContrastArgs(C.Structure):
+    """scde_b200_contrast_args (include/scde_b200.h)."""
+    _fields_ = [
+        ("n_groups", C.c_int32), ("group_offsets", i32p), ("group_cells", i32p),
+        ("n_contrasts", C.c_int32), ("pairs", i32p),
+        ("n_boot", C.c_int32), ("seed", C.c_int32),
+        ("zero_index", i32p), ("n_zero", C.c_int32), ("zero_index_adjusted", i32p),
+        ("batch", i32p), ("n_batch_levels", C.c_int32),
+        ("batch_models", f64p), ("batch_local_theta", C.c_int32), ("batch_square_logit_conc", C.c_int32),
+    ]
+
+
+class ContrastOut(C.Structure):
+    """scde_b200_contrast_out (include/scde_b200.h)."""
+    _fields_ = [
+        ("idx", i32p), ("z", f64p), ("cz", f64p),
+        ("batch_idx", i32p), ("batch_z", f64p), ("batch_cz", f64p),
+        ("adjusted_idx", i32p), ("adjusted_z", f64p), ("adjusted_cz", f64p),
+        ("difference_posterior", f64p), ("adjusted_difference_posterior", f64p), ("joint_posteriors", f64p),
+    ]
+
+
 class Stats(C.Structure):
     _fields_ = [("ms", C.c_float * T_COUNT), ("launches", C.c_int32 * T_COUNT),
                 ("table_rows", C.c_int64), ("contract_cells", C.c_int64)]
@@ -79,7 +110,8 @@ EXPORTED = [
     "scde_b200_bh_cz", "scde_b200_expression_difference", "scde_b200_diff_upload", "scde_b200_diff_run",
     "scde_b200_diff_download", "scde_b200_diff_free", "scde_b200_expression_magnitude", "scde_b200_cell_table",
     "scde_b200_measure_fp64_peak", "scde_b200_set_contract_kernel", "scde_b200_probe_contract_i8",
-    "scde_b200_failure_probability", "scde_b200_expression_prior",
+    "scde_b200_failure_probability", "scde_b200_expression_prior", "scde_b200_dataset_create",
+    "scde_b200_dataset_contrasts", "scde_b200_dataset_free",
 ]
 
 _lib = None
@@ -112,6 +144,11 @@ def lib():
         L.scde_b200_failure_probability.argtypes = [C.c_void_p, f64p, C.c_int32, i32p, f64p, C.c_int32, C.c_int32, f64p]
         L.scde_b200_expression_prior.argtypes = [C.c_void_p, f64p, C.c_int32, i32p, C.c_int32, C.c_int32, C.c_int32,
                                                  C.c_double, C.c_double, C.c_double, C.c_double, f64p, f64p, f64p, f64p]
+        L.scde_b200_dataset_create.argtypes = [C.c_void_p, C.POINTER(DatasetArgs), C.POINTER(C.c_void_p), C.POINTER(Stats)]
+        L.scde_b200_dataset_contrasts.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(ContrastArgs), C.POINTER(ContrastOut),
+                                                  C.POINTER(Stats)]
+        L.scde_b200_dataset_free.argtypes = [C.c_void_p, C.c_void_p]
+        L.scde_b200_dataset_free.restype = None
         L.scde_b200_create_multi.argtypes = [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_void_p)]
         L.scde_b200_n_devices.argtypes = [C.c_void_p]
         L.scde_b200_get_options.argtypes = [C.c_void_p, C.POINTER(Options)]

@@ -627,3 +627,229 @@ def scde_test_gene_expression_difference(gene, models: pd.DataFrame, counts: pd.
     if return_details:
         return {"results": rep, "difference.posterior": bdiffp, "posteriors": {glev[i]: jpl[i] for i in range(2)}}
     return rep
+
+
+# ------------------------------------------------------------------------------------------------
+# many contrasts on one resident dataset
+def _side_label(levels: Sequence) -> str:
+    return str(levels[0]) if len(levels) == 1 else "+".join(str(v) for v in levels)
+
+
+def expand_contrasts(levels: Sequence, contrasts="pairs") -> list:
+    """The contrasts of a call as ``(label, levels of A, levels of B, name of A, name of B)``, A the first level of the
+    two-level factor each contrast stands for (a positive fold change = higher in A).
+
+    ``"pairs"``: every (a, b) with a before b in level order; ``"rest"``: every level against the union of the others,
+    B named ``"rest"``; otherwise a list of (A, B), each side a level name or a list of level names (their union).
+    The labels are ``"<A> vs <B>"`` with a union written ``a+b``.  Host only."""
+    levels = list(levels)
+    out = []
+    if isinstance(contrasts, str):
+        if contrasts not in ("pairs", "rest"):
+            _stop(f'contrasts must be "pairs", "rest" or a list of pairs, not "{contrasts}"')
+        if len(levels) < 2:
+            _stop("the grouping factor needs at least two levels to compare")
+        if contrasts == "pairs":
+            for i, a in enumerate(levels):
+                for b in levels[i + 1:]:
+                    out.append((f"{a} vs {b}", [a], [b], str(a), str(b)))
+        else:
+            for a in levels:
+                rest = [b for b in levels if b != a]
+                out.append((f"{a} vs rest", [a], rest, str(a), "rest"))
+        return out
+    pairs = list(contrasts)
+    if not pairs:
+        _stop("no contrasts given")
+    for pair in pairs:
+        if isinstance(pair, str) or len(pair) != 2:
+            _stop("each contrast must be a pair (A, B) of level names or lists of level names")
+        sides = []
+        for side in pair:
+            lv = [side] if isinstance(side, str) or not isinstance(side, (list, tuple, set, np.ndarray)) else list(side)
+            if not lv:
+                _stop("a side of a contrast names no level")
+            for v in lv:
+                if v not in levels:
+                    _stop(f"unknown level {v} in a contrast (levels: " + " ".join(map(str, levels)) + ")")
+            if len(set(lv)) != len(lv):
+                _stop("a side of a contrast names a level twice")
+            sides.append(lv)
+        if set(sides[0]) & set(sides[1]):
+            _stop("the two sides of a contrast share level(s) " + " ".join(map(str, sorted(set(sides[0]) & set(sides[1]), key=str))))
+        na, nb = _side_label(sides[0]), _side_label(sides[1])
+        out.append((f"{na} vs {nb}", sides[0], sides[1], na, nb))
+    labels = [c[0] for c in out]
+    if len(set(labels)) != len(labels):
+        _stop("a contrast is listed twice")
+    return out
+
+
+class DifferenceSession:
+    """scde.expression.difference for many contrasts over one set of cells.
+
+    The count matrix, its unique-count index and the log-posterior table of every cell stay on the device until
+    ``close()``; each ``contrasts()`` call computes every named group's joint posterior once and all requested contrasts
+    from them.  Every contrast equals ``scde_expression_difference`` called with the corresponding two-level factor (the
+    cells of neither side NA).  While a session is open, the one-shot call on the same context is refused.
+    """
+
+    def __init__(self, models: pd.DataFrame, counts, prior, context=None):
+        self.models = models
+        cm, self.genes = _counts_for_models(models, counts)
+        mm, self._lt, self._sq = pack_models(models)
+        self._x = f64(np.asarray(prior["x"], dtype=np.float64))
+        self._y = f64(np.asarray(prior["y"], dtype=np.float64))
+        with np.errstate(over="ignore"):
+            self._kcols = ["%.15g" % v for v in np.exp(marginals_from_prior(prior))]
+        self.ctx = context or _lib.default_context()
+        self.G, self.C, self.K = cm.shape[0], cm.shape[1], len(self._x)
+        a = _lib.DatasetArgs()
+        a.n_genes, a.n_cells, a.n_grid = self.G, self.C, self.K
+        a.counts, a.models, a.prior_x, a.prior_y = p_i32(cm), p_f64(mm), p_f64(self._x), p_f64(self._y)
+        a.local_theta, a.square_logit_conc = self._lt, self._sq
+        self._ds = C.c_void_p()
+        st = _lib.Stats()
+        check(lib().scde_b200_dataset_create(self.ctx.handle, C.byref(a), C.byref(self._ds), C.byref(st)))
+        self.create_stats = st.as_dict()
+        self.last_stats = None
+
+    def contrasts(self, groups, contrasts="pairs", batch=None, batch_models=None, n_randomizations: int = 150,
+                  return_posteriors: bool = False, expectation=0, seed: int = 1) -> dict:
+        """``{"<A> vs <B>": result}``, each result what ``scde_expression_difference`` returns for that contrast."""
+        if not self._ds:
+            _stop("the session is closed")
+        gcodes, glev = _named_factor(groups, self.models.index)
+        plan = expand_contrasts(glev, contrasts)
+        code_of = {lev: i for i, lev in enumerate(glev)}
+        sides, side_id, pairs = [], {}, []
+        for label, la, lb, _na, _nb in plan:
+            ids = []
+            for lv in (la, lb):
+                key = tuple(sorted(code_of[v] for v in lv))
+                if key not in side_id:
+                    cells = np.nonzero(np.isin(gcodes, key))[0].astype(np.int32)
+                    if len(cells) == 0:
+                        _stop(f"no cells in {_side_label(lv)} (contrast {label})")
+                    side_id[key] = len(sides)
+                    sides.append(cells)
+                ids.append(side_id[key])
+            pairs += ids
+        correct_batch, bcodes, blev = False, None, []
+        if batch is not None:
+            bcodes, blev = _named_factor(batch, self.models.index)
+            correct_batch = len(blev) > 1
+        bmm, blt, bsq = None, 0, 0
+        if correct_batch and batch_models is not None and batch_models is not self.models:
+            if list(batch_models.index) != list(self.models.index):
+                if not all(c in batch_models.index for c in self.models.index):
+                    _stop("batch.models does not cover all of the cells specified in the model matrix")
+                batch_models = batch_models.loc[list(self.models.index)]
+            bmm, blt, bsq = pack_models(batch_models)
+        if correct_batch:  # the warning of R/functions.R:336-349, per contrast
+            for label, la, lb, _na, _nb in plan:
+                ia, ib = (sides[side_id[tuple(sorted(code_of[v] for v in lv))]] for lv in (la, lb))
+                tab = np.array([np.bincount(bcodes[i][bcodes[i] >= 0], minlength=len(blev)) for i in (ia, ib)])
+                pval = fisher_test_p_value(tab)
+                if pval < 1e-3:
+                    sys.stdout.write(f"WARNING: strong interaction between groups and batches in {label}! "
+                                     "Correction may be ineffective:\n")
+                    sys.stdout.write(f"Fisher's Exact Test for Count Data: p-value = {pval:.4g}\n")
+        diffv = fold_change_grid(self._x)
+        zi = _zero_index(diffv, expectation)
+        if len(zi) not in (1, self.G):
+            _stop("the expectation parameter must be either one number or a vector equal to the number of genes being tested")
+        adiffv = r_as_character_numeric(r_seq_length(diffv[0] - diffv[-1], diffv[-1] - diffv[0], 2 * len(diffv) - 1))
+        zia = _zero_index(adiffv, expectation)
+        nc, ng, G, K = len(plan), len(sides), self.G, self.K
+        off = np.zeros(ng + 1, dtype=np.int32)
+        off[1:] = np.cumsum([len(s) for s in sides])
+        cells = np.concatenate(sides).astype(np.int32)
+        pr = np.asarray(pairs, dtype=np.int32)
+        a = _lib.ContrastArgs()
+        a.n_groups, a.group_offsets, a.group_cells = ng, p_i32(off), p_i32(cells)
+        a.n_contrasts, a.pairs = nc, p_i32(pr)
+        a.n_boot, a.seed = int(n_randomizations), int(seed)
+        zi, zia = i32(zi), i32(zia)
+        a.zero_index, a.n_zero, a.zero_index_adjusted = p_i32(zi), len(zi), p_i32(zia)
+        bc = i32(bcodes) if correct_batch else None
+        a.batch, a.n_batch_levels = p_i32(bc), len(blev) if correct_batch else 0
+        if bmm is not None:
+            a.batch_models, a.batch_local_theta, a.batch_square_logit_conc = p_f64(bmm), blt, bsq
+        o = _lib.ContrastOut()
+        r = {"idx": np.empty((nc, 3, G), np.int32), "z": np.empty((nc, G)), "cz": np.empty((nc, G))}
+        o.idx, o.z, o.cz = p_i32(r["idx"]), p_f64(r["z"]), p_f64(r["cz"])
+        if correct_batch:
+            for k in ("batch", "adjusted"):
+                r[k + "_idx"], r[k + "_z"], r[k + "_cz"] = np.empty((nc, 3, G), np.int32), np.empty((nc, G)), np.empty((nc, G))
+                setattr(o, k + "_idx", p_i32(r[k + "_idx"]))
+                setattr(o, k + "_z", p_f64(r[k + "_z"]))
+                setattr(o, k + "_cz", p_f64(r[k + "_cz"]))
+        if return_posteriors:
+            r["post"] = np.empty((nc, 2 * K - 1, G))
+            r["jp"] = np.empty((ng, K, G))
+            o.difference_posterior, o.joint_posteriors = p_f64(r["post"]), p_f64(r["jp"])
+            if correct_batch:
+                r["apost"] = np.empty((nc, 4 * K - 3, G))
+                o.adjusted_difference_posterior = p_f64(r["apost"])
+        st = _lib.Stats()
+        check(lib().scde_b200_dataset_contrasts(self.ctx.handle, self._ds, C.byref(a), C.byref(o), C.byref(st)))
+        self.last_stats = st.as_dict()
+        genes = self.genes
+        out = {}
+        for c, (label, la, lb, na, nb) in enumerate(plan):
+            res = _summary_frame(r["idx"][c].T, r["z"][c], diffv, genes, cz=r["cz"][c])
+            posts = {}
+            if return_posteriors:
+                ja, jb = pairs[2 * c], pairs[2 * c + 1]
+                posts = {"difference.posterior": pd.DataFrame(r["post"][c].T, index=genes, columns=["%.15g" % v for v in diffv]),
+                         "joint.posteriors": {na: pd.DataFrame(r["jp"][ja].T, index=genes, columns=self._kcols),
+                                              nb: pd.DataFrame(r["jp"][jb].T, index=genes, columns=self._kcols)}}
+            if correct_batch:
+                d = {"batch.adjusted": _summary_frame(r["adjusted_idx"][c].T, r["adjusted_z"][c], adiffv, genes,
+                                                      cz=r["adjusted_cz"][c]),
+                     "results": res,
+                     "batch.effect": _summary_frame(r["batch_idx"][c].T, r["batch_z"][c], diffv, genes, cz=r["batch_cz"][c])}
+                if return_posteriors:
+                    d.update(posts)
+                    d["batch.adjusted.difference.posterior"] = pd.DataFrame(
+                        r["apost"][c].T, index=genes, columns=["%.15g" % v for v in adiffv])
+                d["stats"] = self.last_stats
+                out[label] = d
+            elif return_posteriors:
+                d = {"results": res}
+                d.update(posts)
+                d["stats"] = self.last_stats
+                out[label] = d
+            else:
+                res.attrs["stats"] = self.last_stats
+                out[label] = res
+        return out
+
+    def close(self):
+        if getattr(self, "_ds", None):
+            lib().scde_b200_dataset_free(self.ctx.handle, self._ds)
+            self._ds = C.c_void_p()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def scde_expression_difference_contrasts(models: pd.DataFrame, counts, prior, groups, contrasts="pairs", batch=None,
+                                         batch_models=None, n_randomizations: int = 150, return_posteriors: bool = False,
+                                         expectation=0, seed: int = 1, context=None) -> dict:
+    """scde.expression.difference for every contrast of `groups` (``"pairs"``, ``"rest"`` or a list of pairs; see
+    ``expand_contrasts``) in one device session: ``{"<A> vs <B>": result}``."""
+    with DifferenceSession(models, counts, prior, context=context) as s:
+        return s.contrasts(groups, contrasts=contrasts, batch=batch, batch_models=batch_models,
+                           n_randomizations=n_randomizations, return_posteriors=return_posteriors,
+                           expectation=expectation, seed=seed)

@@ -11,6 +11,9 @@
 #include <cstring>
 #include <string>
 #include <chrono>
+#include <exception>
+#include <map>
+#include <new>
 #include <thread>
 #include <vector>
 
@@ -2064,13 +2067,14 @@ struct OutPlace {
     int64_t ld, row0;
 };
 
-static int download_matrix(scde_b200_ctx *ctx, scde_b200_diff_job *j, const double *src, int ld_src, int cols, double *dst,
+// [G][ld_src] gene-major device matrix -> rows row0.. of a column-major host matrix with pl.ld rows
+static int download_matrix(scde_b200_ctx *ctx, DiffWorkspace *ws, int G, const double *src, int ld_src, int cols, double *dst,
                            OutPlace pl) {
     cudaStream_t st = ctx->stream;
-    SCDE_CUDA(j->ws->tbuf.ensure((size_t)j->G * cols));
-    SCDE_CUDA(launch_transpose_out(src, ld_src, j->G, cols, j->ws->tbuf.p, st));
-    SCDE_CUDA(cudaMemcpy2DAsync(dst + pl.row0, sizeof(double) * (size_t)pl.ld, j->ws->tbuf.p, sizeof(double) * (size_t)j->G,
-                                sizeof(double) * (size_t)j->G, cols, cudaMemcpyDeviceToHost, st));
+    SCDE_CUDA(ws->tbuf.ensure((size_t)G * cols));
+    SCDE_CUDA(launch_transpose_out(src, ld_src, G, cols, ws->tbuf.p, st));
+    SCDE_CUDA(cudaMemcpy2DAsync(dst + pl.row0, sizeof(double) * (size_t)pl.ld, ws->tbuf.p, sizeof(double) * (size_t)G,
+                                sizeof(double) * (size_t)G, cols, cudaMemcpyDeviceToHost, st));
     SCDE_CUDA(cudaStreamSynchronize(st));
     return SCDE_B200_OK;
 }
@@ -2130,25 +2134,25 @@ static int diff_download_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, const s
         }
         SCDE_CUDA(cudaStreamSynchronize(st));
         for (int i = 0; i < 2; ++i) {
-            if (o->joint_posteriors[i]) TRY(download_matrix(ctx, j, j->ws->jp[i].p, ld, K, o->joint_posteriors[i], pl));
+            if (o->joint_posteriors[i]) TRY(download_matrix(ctx, j->ws, j->G, j->ws->jp[i].p, ld, K, o->joint_posteriors[i], pl));
             if (j->has_batch && o->batch_joint_posteriors[i])
-                TRY(download_matrix(ctx, j, j->ws->jp[2 + i].p, ld, K, o->batch_joint_posteriors[i], pl));
+                TRY(download_matrix(ctx, j->ws, j->G, j->ws->jp[2 + i].p, ld, K, o->batch_joint_posteriors[i], pl));
         }
         if (o->difference_posterior) {
             if (!j->ws->post.p) {
                 set_error("difference_posterior requested but the job was uploaded without want_posteriors");
                 return SCDE_B200_EINVAL;
             }
-            TRY(download_matrix(ctx, j, j->ws->post.p, ldo, nout, o->difference_posterior, pl));
+            TRY(download_matrix(ctx, j->ws, j->G, j->ws->post.p, ldo, nout, o->difference_posterior, pl));
         }
         if (j->has_batch && o->batch_difference_posterior)
-            TRY(download_matrix(ctx, j, j->ws->bpost.p, ldo, nout, o->batch_difference_posterior, pl));
+            TRY(download_matrix(ctx, j->ws, j->G, j->ws->bpost.p, ldo, nout, o->batch_difference_posterior, pl));
         if (j->has_batch && o->adjusted_difference_posterior) {
             if (!j->ws->apost.p) {
                 set_error("adjusted posterior requested but the job was uploaded without want_posteriors");
                 return SCDE_B200_EINVAL;
             }
-            TRY(download_matrix(ctx, j, j->ws->apost.p, lda, nadj, o->adjusted_difference_posterior, pl));
+            TRY(download_matrix(ctx, j->ws, j->G, j->ws->apost.p, lda, nadj, o->adjusted_difference_posterior, pl));
         }
     }
     SCDE_CUDA(cudaStreamSynchronize(st));
@@ -2278,6 +2282,680 @@ int scde_b200_expression_difference(scde_b200_ctx *ctx, const scde_b200_diff_arg
     if (has_batch && out->batch_cz) scde::bh_cz(out->batch_z, n, out->batch_cz);
     if (has_batch && out->adjusted_cz) scde::bh_cz(out->adjusted_z, n, out->adjusted_cz);
     return SCDE_B200_OK;
+}
+
+}  // extern "C"
+
+// ============================================================================================
+// Many contrasts on one resident dataset.  The index and the table cover every cell, so they do not depend on the grouping;
+// a group's joint depends only on its cells, the seed, n_boot and (through the draws) its size, because every
+// scde.posteriors call of the reference re-seeds srand(Seed); a batch joint depends only on the composition of its group.
+// A call therefore computes each named group's joint once into a bank slot, each distinct composition's batch joint once,
+// and runs the ratio and summary passes of all contrasts in batched launches on the bank.
+
+namespace {
+
+// The host part of one contrasts call, shared by the per-device shards: which joints exist and which draws they use.
+struct ContrastPlan {
+    int C = 0, K = 0, N = 0;          // cells, grid points, genes of the dataset
+    int n_contrasts = 0, n_boot = 0;
+    bool has_batch = false, want_post = false;
+    std::vector<int> slot_group;      // bank slot -> group id (only groups some contrast names)
+    std::vector<int32_t> cells;       // the slots' cells back to back
+    std::vector<int64_t> cell_off;    // slot -> offset into cells (n_slots + 1)
+    std::vector<int32_t> draws;       // group draws, one set per distinct group size
+    std::vector<int64_t> draw_off;    // slot -> offset into draws
+    std::vector<int> bslot_D;         // batch slot (distinct composition) -> draws per boot
+    std::vector<int32_t> bdraws;      // batch draws (global cell ids), one set per batch slot
+    std::vector<int64_t> bdraw_off;
+    std::vector<int> pair_slot, pair_bslot;  // 2 per contrast
+    std::vector<int32_t> zi, zi_adj;  // n_zero entries each (1 or N)
+    int n_zero = 1;
+    const double *batch_models = nullptr;
+    int b_local_theta = 0, b_sqlogit = 0;
+    bool b_fast_theta = false;
+};
+
+}  // namespace
+
+// one device's part of a dataset: genes [g0, g0 + G)
+struct DatasetShard {
+    scde_b200_ctx *ctx = nullptr;
+    int g0 = 0, G = 0, C = 0, K = 0;
+    int local_theta = 0, sqlogit = 0;
+    bool fast_theta = false;
+    DiffWorkspace *ws = nullptr;
+    DBuf<double> models, mag, prior_y, bmodels;
+    // what the table rows hold: built from `models` (0) or from a call's batch.models (1), for the tcgen05 kernel
+    // (fixed-point planes) or the FP64 kernels (FP64 rows)
+    int rows_from = 0;
+    bool rows_i8 = false;
+    DBuf<double> bank, bbank;                 // joint posteriors, [slot][G][ld]
+    DBuf<int32_t> cells, draws, bdraws, zi, zi_adj, jflags;
+    DBuf<int32_t> idx, bidx, aidx;            // [contrast][3][G]
+    DBuf<double> z, bz, az;                   // [contrast][G]
+    DBuf<RatioContrast> rtab;                 // [pass][contrast] device tables of the batched ratio launches
+    StageTimer timer;
+    ~DatasetShard() {
+        if (ctx) {
+            cudaSetDevice(ctx->device);
+            ctx->ws_busy = false;
+        }
+    }
+};
+
+struct scde_b200_dataset {
+    scde_b200_ctx *owner = nullptr;
+    int n_genes = 0, n_cells = 0, n_grid = 0;
+    std::vector<DatasetShard *> shards;
+    ~scde_b200_dataset() {
+        for (auto *s : shards) delete s;
+    }
+};
+
+namespace {
+
+// rebuild the table rows from the models (from_batch = 0) or from the call's batch.models (1) for the kernel the context
+// selects now, unless they already are
+int ensure_rows(DatasetShard &sh, const ContrastPlan &p, int from_batch, StageTimer *tm) {
+    scde_b200_ctx *ctx = sh.ctx;
+    LpTable &t = sh.ws->table;
+    const bool i8 = want_i8(ctx);
+    if (sh.rows_from == from_batch && sh.rows_i8 == i8 && !from_batch) return SCDE_B200_OK;
+    t.want_q = i8;
+    sh.rows_from = -1;  // unknown until the rebuild has been queued
+    if (from_batch) {
+        t.fast_theta = p.b_fast_theta;
+        const int r = fill_table(ctx, t, sh.bmodels.p, sh.C, sh.mag.p, p.b_local_theta, p.b_sqlogit, tm);
+        t.fast_theta = sh.fast_theta;
+        TRY(r);
+    } else {
+        TRY(fill_table(ctx, t, sh.models.p, sh.C, sh.mag.p, sh.local_theta, sh.sqlogit, tm));
+    }
+    sh.rows_from = from_batch;
+    sh.rows_i8 = i8;
+    return SCDE_B200_OK;
+}
+
+int shard_create(scde_b200_ctx *ctx, const scde_b200_dataset_args *a, int g0, int g1, DatasetShard **out) {
+    CHECK_CTX(ctx);
+    *out = nullptr;
+    if (ctx->ws_busy) {
+        set_error("another expression_difference job is alive on this context (free it first)");
+        return SCDE_B200_EINVAL;
+    }
+    if (!ctx->ws) ctx->ws = new DiffWorkspace();
+    DatasetShard *sh = new DatasetShard();
+    sh->ctx = ctx;  // from here on, deleting the shard releases the workspace
+    ctx->ws_busy = true;
+    sh->ws = ctx->ws;
+    const int G = g1 - g0, C = a->n_cells, K = a->n_grid;
+    sh->g0 = g0;
+    sh->G = G;
+    sh->C = C;
+    sh->K = K;
+    sh->local_theta = a->local_theta;
+    sh->sqlogit = a->square_logit_conc;
+    sh->fast_theta = !a->local_theta && theta_all_regular(a->models, C, C);
+    cudaStream_t st = ctx->stream;
+    auto body = [&]() -> int {
+        SCDE_CUDA(sh->ws->counts.ensure((size_t)G * C));
+        SCDE_CUDA(cudaMemcpy2DAsync(sh->ws->counts.p, sizeof(int32_t) * G, a->counts + g0, sizeof(int32_t) * (size_t)a->n_genes,
+                                    sizeof(int32_t) * G, C, cudaMemcpyHostToDevice, st));
+        TRY(upload(sh->models, a->models, (size_t)C * 12, st));
+        TRY(upload(sh->prior_y, a->prior_y, (size_t)K, st));
+        std::vector<double> mag(K);
+        for (int k = 0; k < K; ++k) {  // R/functions.R:575-577
+            double m = std::pow(10.0, a->prior_x[k]) - 1;
+            if (m < 0) m = 0;
+            mag[k] = std::log(m);
+        }
+        TRY(upload(sh->mag, mag.data(), (size_t)K, st));
+        LpTable &t = sh->ws->table;
+        t.K = K;
+        t.ld = table_ld(K);
+        t.sentinel = -DBL_MAX / C / 1.1;
+        t.fast_theta = sh->fast_theta;
+        t.zero_base = t.ld <= KP_TILED && ctx->opt.zero_base;
+        t.want_q = want_i8(ctx);
+        t.want_modes = false;
+        StageTimer &tm = sh->timer;
+        tm.reset();
+        const int t_all = tm.begin(st);
+        TRY(index_from_counts(ctx, t, sh->ws->counts.p, G, 0, G, C, &tm));
+        TRY(fill_table(ctx, t, sh->models.p, C, sh->mag.p, sh->local_theta, sh->sqlogit, &tm));
+        tm.end(SCDE_B200_T_TOTAL, t_all, st, 0);
+        sh->rows_from = 0;
+        sh->rows_i8 = t.want_q;
+        SCDE_CUDA(cudaStreamSynchronize(st));
+        return SCDE_B200_OK;
+    };
+    const int r = body();
+    if (r != SCDE_B200_OK) {
+        cudaStreamSynchronize(st);
+        delete sh;
+        return r;
+    }
+    *out = sh;
+    return SCDE_B200_OK;
+}
+
+int shard_contrasts(DatasetShard &sh, const ContrastPlan &p, const scde_b200_contrast_out *o, scde_b200_stats *stats) {
+    scde_b200_ctx *ctx = sh.ctx;
+    CHECK_CTX(ctx);
+    cudaStream_t st = ctx->stream;
+    DiffWorkspace *ws = sh.ws;
+    LpTable &t = ws->table;
+    StageTimer &tm = sh.timer;
+    tm.reset();
+    const int G = sh.G, K = sh.K, nc = p.n_contrasts;
+    const int ld = t.ld, nout = 2 * K - 1, ldo = round_up(nout, 8), nadj = 2 * nout - 1, lda = round_up(nadj, 8);
+    const int n_slots = (int)p.slot_group.size(), n_bslots = (int)p.bslot_D.size();
+    SCDE_CUDA(ws->scr.total.ensure(1));
+    SCDE_CUDA(cudaMemsetAsync(ws->scr.total.p, 0, sizeof(unsigned long long), st));
+    const int t_all = tm.begin(st);
+    TRY(ensure_rows(sh, p, 0, &tm));
+    TRY(upload(sh.cells, p.cells.data(), p.cells.size(), st));
+    TRY(upload(sh.draws, p.draws.data(), p.draws.size(), st));
+    if (p.has_batch) TRY(upload(sh.bdraws, p.bdraws.data(), p.bdraws.size(), st));
+    {
+        std::vector<int32_t> zi(p.n_zero == 1 ? 1 : G);
+        for (size_t i = 0; i < zi.size(); ++i) zi[i] = p.zi[p.n_zero == 1 ? 0 : sh.g0 + i];
+        TRY(upload(sh.zi, zi.data(), zi.size(), st));
+        if (p.has_batch) {
+            for (size_t i = 0; i < zi.size(); ++i) zi[i] = p.zi_adj[p.n_zero == 1 ? 0 : sh.g0 + i];
+            TRY(upload(sh.zi_adj, zi.data(), zi.size(), st));
+        }
+        SCDE_CUDA(cudaStreamSynchronize(st));  // the host vectors above go out of scope
+    }
+    if (p.has_batch && p.batch_models) TRY(upload(sh.bmodels, p.batch_models, (size_t)sh.C * 12, st));
+    const size_t slot_sz = (size_t)G * ld;
+    SCDE_CUDA(sh.bank.ensure((size_t)n_slots * slot_sz));
+    if (p.has_batch) SCDE_CUDA(sh.bbank.ensure((size_t)n_bslots * slot_sz));
+    // the tcgen05 kernel's status word, per joint: a joint that raises it is recomputed alone on the FP64 kernel below
+    const int n_joints = n_slots + n_bslots;
+    SCDE_CUDA(sh.jflags.ensure((size_t)n_joints));
+    SCDE_CUDA(cudaMemsetAsync(sh.jflags.p, 0, sizeof(int32_t) * n_joints, st));
+    auto group_joint = [&](int s, bool count) {
+        const int n = (int)(p.cell_off[s + 1] - p.cell_off[s]);
+        return run_joint(ctx, t, sh.cells.p + p.cell_off[s], n, sh.draws.p + p.draw_off[s], p.n_boot, n, (double)p.n_boot,
+                         sh.bank.p + s * slot_sz, ld, ws->scr, &tm, count);
+    };
+    auto batch_joint = [&](int b, bool count, const TwinJoint *tw, bool *twin_done) {
+        return run_joint(ctx, t, nullptr, sh.C, sh.bdraws.p + p.bdraw_off[b], p.n_boot, p.bslot_D[b], (double)p.n_boot,
+                         sh.bbank.p + b * slot_sz, ld, ws->scr, &tm, count, tw, twin_done);
+    };
+    auto keep_flag = [&](int i) {
+        return cudaMemcpyAsync(sh.jflags.p + i, ctx->flags.p, sizeof(int32_t), cudaMemcpyDeviceToDevice, st);
+    };
+    for (int s = 0; s < n_slots; ++s) {
+        TRY(reset_flags(ctx));
+        TRY(group_joint(s, true));
+        SCDE_CUDA(keep_flag(s));
+    }
+    if (p.has_batch) {
+        if (p.batch_models) TRY(ensure_rows(sh, p, 1, &tm));
+        // distinct compositions in pairs: one launch of the tcgen05 kernel for two joints over the same cells and rows
+        for (int b = 0; b < n_bslots; b += 2) {
+            TRY(reset_flags(ctx));
+            bool twin_done = false;
+            if (b + 1 < n_bslots) {
+                TwinJoint tw{sh.bdraws.p + p.bdraw_off[b + 1], p.bslot_D[b + 1], sh.bbank.p + (b + 1) * slot_sz, &ws->scr2};
+                TRY(batch_joint(b, true, &tw, &twin_done));
+                if (!twin_done) TRY(batch_joint(b + 1, true, nullptr, nullptr));
+                SCDE_CUDA(keep_flag(n_slots + b + 1));
+            } else {
+                TRY(batch_joint(b, true, nullptr, nullptr));
+            }
+            SCDE_CUDA(keep_flag(n_slots + b));
+        }
+    }
+    std::vector<int32_t> flags(n_joints);
+    SCDE_CUDA(cudaMemcpyAsync(flags.data(), sh.jflags.p, sizeof(int32_t) * n_joints, cudaMemcpyDeviceToHost, st));
+    SCDE_CUDA(cudaStreamSynchronize(st));
+    bool any = false;
+    for (int f : flags) {
+        if (f & 2) {
+            set_error("tcgen05 contraction kernel aborted (pipeline watchdog); use scde_b200_set_contract_kernel(ctx, 2)");
+            return SCDE_B200_ECUDA;
+        }
+        any = any || (f & (1 | 4));
+    }
+    if (any) {  // only the flagged joints are repeated, on the FP64 kernel (FP64 table rows)
+        const int keep = ctx->opt.contract_kernel;
+        ctx->opt.contract_kernel = 2;
+        auto rerun = [&]() -> int {
+            bool rows = false;
+            for (int s = 0; s < n_slots; ++s)
+                if (flags[s] & (1 | 4)) {
+                    if (!rows) TRY(ensure_rows(sh, p, 0, &tm));
+                    rows = true;
+                    TRY(group_joint(s, false));
+                }
+            rows = false;
+            for (int b = 0; b < n_bslots; ++b)
+                if (flags[n_slots + b] & (1 | 4)) {
+                    if (!rows) TRY(ensure_rows(sh, p, p.batch_models ? 1 : 0, &tm));
+                    rows = true;
+                    TRY(batch_joint(b, false, nullptr, nullptr));
+                }
+            return SCDE_B200_OK;
+        };
+        const int r = rerun();
+        ctx->opt.contract_kernel = keep;
+        TRY(r);
+    }
+    // ratio and summary: every contrast in one launch per pass; the 2K-1 posteriors that feed the adjusted pass (or that
+    // the caller wants) exist only for a block of contrasts at a time, sized to the free device memory
+    const bool keep_post = p.want_post || p.has_batch;
+    SCDE_CUDA(sh.idx.ensure((size_t)nc * 3 * G));
+    SCDE_CUDA(sh.z.ensure((size_t)nc * G));
+    if (p.has_batch) {
+        SCDE_CUDA(sh.bidx.ensure((size_t)nc * 3 * G));
+        SCDE_CUDA(sh.bz.ensure((size_t)nc * G));
+        SCDE_CUDA(sh.aidx.ensure((size_t)nc * 3 * G));
+        SCDE_CUDA(sh.az.ensure((size_t)nc * G));
+    }
+    int nb = nc;
+    if (keep_post) {
+        const size_t per = sizeof(double) * (size_t)G * ((p.has_batch ? 2 : 1) * (size_t)ldo + (p.want_post && p.has_batch ? lda : 0));
+        size_t free_b = 0, total_b = 0;
+        SCDE_CUDA(cudaMemGetInfo(&free_b, &total_b));
+        const size_t have = sizeof(double) * (ws->post.cap + ws->bpost.cap + ws->apost.cap);
+        const size_t fit = (free_b / 2 + have) / per;
+        nb = fit < 1 ? 1 : (fit < (size_t)nc ? (int)fit : nc);
+        SCDE_CUDA(ws->post.ensure((size_t)nb * G * ldo));
+        if (p.has_batch) SCDE_CUDA(ws->bpost.ensure((size_t)nb * G * ldo));
+        if (p.has_batch && p.want_post) SCDE_CUDA(ws->apost.ensure((size_t)nb * G * lda));
+    }
+    const int n_pass = p.has_batch ? 3 : 1;
+    std::vector<RatioContrast> tab((size_t)n_pass * nc);
+    for (int c = 0; c < nc; ++c) {
+        const size_t k = (size_t)(c % nb);
+        RatioContrast &m = tab[c];
+        m.p1 = sh.bank.p + p.pair_slot[2 * c] * slot_sz;
+        m.p2 = sh.bank.p + p.pair_slot[2 * c + 1] * slot_sz;
+        m.idx = sh.idx.p + (size_t)c * 3 * G;
+        m.z = sh.z.p + (size_t)c * G;
+        m.post = keep_post ? ws->post.p + k * G * ldo : nullptr;
+        if (!p.has_batch) continue;
+        RatioContrast &b = tab[nc + c];
+        b.p1 = sh.bbank.p + p.pair_bslot[2 * c] * slot_sz;
+        b.p2 = sh.bbank.p + p.pair_bslot[2 * c + 1] * slot_sz;
+        b.idx = sh.bidx.p + (size_t)c * 3 * G;
+        b.z = sh.bz.p + (size_t)c * G;
+        b.post = ws->bpost.p + k * G * ldo;
+        RatioContrast &a = tab[2 * nc + c];
+        a.p1 = m.post;
+        a.p2 = b.post;
+        a.idx = sh.aidx.p + (size_t)c * 3 * G;
+        a.z = sh.az.p + (size_t)c * G;
+        a.post = p.want_post ? ws->apost.p + k * G * lda : nullptr;
+    }
+    TRY(upload(sh.rtab, tab.data(), tab.size(), st));
+    const int64_t N = p.N;
+    for (int c0 = 0; c0 < nc; c0 += nb) {
+        const int n = nc - c0 < nb ? nc - c0 : nb;
+        const int e0 = tm.begin(st);
+        RatioArgs r{};
+        r.ld = ld;
+        r.n_genes = G;
+        r.n = K;
+        r.prior = sh.prior_y.p;
+        r.zero_index = sh.zi.p;
+        r.n_zero = p.n_zero == 1 ? 1 : G;
+        r.ld_post = ldo;
+        r.contrasts = sh.rtab.p + c0;
+        r.n_contrasts = n;
+        SCDE_CUDA(launch_ratio_summary(r, st));
+        if (p.has_batch) {
+            // batch.effect with the default expectation = 0 (R/functions.R:362): H0 index = centre of the grid
+            RatioArgs b = r;
+            b.zero_index = nullptr;
+            b.n_zero = 1;
+            b.contrasts = sh.rtab.p + nc + c0;
+            SCDE_CUDA(launch_ratio_summary(b, st));
+            // batch adjustment: the two 2K-1 posteriors slid without prior weighting (R/functions.R:391)
+            RatioArgs a{};
+            a.ld = ldo;
+            a.n_genes = G;
+            a.n = nout;
+            a.zero_index = sh.zi_adj.p;
+            a.n_zero = p.n_zero == 1 ? 1 : G;
+            a.ld_post = lda;
+            a.contrasts = sh.rtab.p + 2 * nc + c0;
+            a.n_contrasts = n;
+            SCDE_CUDA(launch_ratio_summary(a, st));
+        }
+        tm.end(SCDE_B200_T_RATIO, e0, st, n_pass);
+        for (int c = c0; c < c0 + n && p.want_post; ++c) {
+            const size_t k = (size_t)(c - c0);
+            if (o->difference_posterior)
+                TRY(download_matrix(ctx, ws, G, ws->post.p + k * G * ldo, ldo, nout, o->difference_posterior + (size_t)c * N * nout,
+                                    OutPlace{N, sh.g0}));
+            if (p.has_batch && o->adjusted_difference_posterior)
+                TRY(download_matrix(ctx, ws, G, ws->apost.p + k * G * lda, lda, nadj,
+                                    o->adjusted_difference_posterior + (size_t)c * N * nadj, OutPlace{N, sh.g0}));
+        }
+    }
+    tm.end(SCDE_B200_T_TOTAL, t_all, st, 0);
+    auto get_idx = [&](int32_t *dst, const int32_t *src) {  // [3][G] -> rows g0.. of the N x 3 block
+        return cudaMemcpy2DAsync(dst + sh.g0, sizeof(int32_t) * (size_t)N, src, sizeof(int32_t) * (size_t)G,
+                                 sizeof(int32_t) * (size_t)G, 3, cudaMemcpyDeviceToHost, st);
+    };
+    auto get_z = [&](double *dst, const double *src) {
+        return cudaMemcpyAsync(dst + sh.g0, src, sizeof(double) * (size_t)G, cudaMemcpyDeviceToHost, st);
+    };
+    for (int c = 0; c < nc; ++c) {
+        const size_t i3 = (size_t)c * 3 * G, i1 = (size_t)c * G, o3 = (size_t)c * 3 * N, o1 = (size_t)c * N;
+        if (o->idx) SCDE_CUDA(get_idx(o->idx + o3, sh.idx.p + i3));
+        if (o->z) SCDE_CUDA(get_z(o->z + o1, sh.z.p + i1));
+        if (!p.has_batch) continue;
+        if (o->batch_idx) SCDE_CUDA(get_idx(o->batch_idx + o3, sh.bidx.p + i3));
+        if (o->batch_z) SCDE_CUDA(get_z(o->batch_z + o1, sh.bz.p + i1));
+        if (o->adjusted_idx) SCDE_CUDA(get_idx(o->adjusted_idx + o3, sh.aidx.p + i3));
+        if (o->adjusted_z) SCDE_CUDA(get_z(o->adjusted_z + o1, sh.az.p + i1));
+    }
+    if (o->joint_posteriors)
+        for (int s = 0; s < n_slots; ++s)
+            TRY(download_matrix(ctx, ws, G, sh.bank.p + s * slot_sz, ld, K,
+                                o->joint_posteriors + (size_t)p.slot_group[s] * N * K, OutPlace{N, sh.g0}));
+    SCDE_CUDA(cudaStreamSynchronize(st));
+    if (stats) {
+        tm.collect(stats);
+        stats->table_rows = t.n_rows;
+        unsigned long long tot = 0;
+        SCDE_CUDA(cudaMemcpy(&tot, ws->scr.total.p, sizeof(tot), cudaMemcpyDeviceToHost));
+        stats->contract_cells = (int64_t)tot;
+    }
+    return SCDE_B200_OK;
+}
+
+// shard i of n over genes [0, N): the split of expression_difference_multi
+void shard_range(int N, int n, int i, int *b, int *e) {
+    const int base = N / n, rem = N % n;
+    *b = i * base + (i < rem ? i : rem);
+    *e = *b + base + (i < rem ? 1 : 0);
+}
+
+// Runs f(i) for i < n on one host thread each (directly when n == 1); exceptions become return codes, the first failing
+// shard's error text becomes this thread's.
+template <class F>
+int on_shards(int n, const std::vector<scde_b200_ctx *> &devs, F f, std::vector<scde_b200_stats> *sst, scde_b200_stats *stats) {
+    std::vector<int> rc(n, SCDE_B200_OK);
+    std::vector<std::string> msg(n);
+    auto body = [&](int i) {
+        try {
+            rc[i] = f(i);
+            if (rc[i] != SCDE_B200_OK) msg[i] = g_err;  // the error text is thread-local
+        } catch (const std::bad_alloc &) {
+            rc[i] = SCDE_B200_ENOMEM;
+            msg[i] = "host allocation failed";
+        } catch (const std::exception &ex) {
+            rc[i] = SCDE_B200_EINVAL;
+            msg[i] = ex.what();
+        } catch (...) {
+            rc[i] = SCDE_B200_EINVAL;
+            msg[i] = "unknown exception";
+        }
+    };
+    if (n == 1) {
+        body(0);
+    } else {
+        std::vector<std::thread> th;
+        try {
+            for (int i = 0; i < n; ++i) th.emplace_back(body, i);
+        } catch (...) {
+            for (auto &t : th) t.join();
+            set_error("could not start a host thread per device");
+            return SCDE_B200_ENOMEM;
+        }
+        for (auto &t : th) t.join();
+    }
+    cudaSetDevice(devs[0]->device);
+    for (int i = 0; i < n; ++i)
+        if (rc[i] != SCDE_B200_OK) {
+            if (n == 1)
+                g_err = msg[i];
+            else
+                set_error("device %d (shard %d of %d): %s", devs[i]->device, i, n, msg[i].c_str());
+            return rc[i];
+        }
+    if (stats && sst) {  // stage times: the slowest shard; counters: summed
+        memset(stats, 0, sizeof(*stats));
+        for (int i = 0; i < n; ++i) {
+            for (int k = 0; k < SCDE_B200_T_COUNT; ++k) {
+                if ((*sst)[i].ms[k] > stats->ms[k]) stats->ms[k] = (*sst)[i].ms[k];
+                stats->launches[k] += (*sst)[i].launches[k];
+            }
+            stats->table_rows += (*sst)[i].table_rows;
+            stats->contract_cells += (*sst)[i].contract_cells;
+        }
+    }
+    return SCDE_B200_OK;
+}
+
+std::vector<scde_b200_ctx *> context_devices(scde_b200_ctx *ctx) {
+    std::vector<scde_b200_ctx *> devs{ctx};
+    for (auto *c : ctx->children) devs.push_back(c);
+    return devs;
+}
+
+// validation of a contrasts call and everything about it that does not depend on the device
+int plan_contrasts(const scde_b200_dataset *ds, const scde_b200_contrast_args *a, const scde_b200_contrast_out *o,
+                   ContrastPlan &p) {
+    const int C = ds->n_cells, K = ds->n_grid, N = ds->n_genes;
+    auto bad = [](const char *fmt, auto... v) {
+        set_error(fmt, v...);
+        return SCDE_B200_EINVAL;
+    };
+    if (a->n_groups < 2 || !a->group_offsets || !a->group_cells) return bad("contrasts: need at least two groups");
+    if (a->n_contrasts < 1 || !a->pairs) return bad("contrasts: need at least one contrast");
+    if (a->n_boot < 1) return bad("contrasts: n_boot must be >= 1");
+    if ((o->cz && !o->z) || (o->batch_cz && !o->batch_z) || (o->adjusted_cz && !o->adjusted_z))
+        return bad("contrasts: a cZ output needs the matching Z output");
+    if (a->group_offsets[0] != 0) return bad("contrasts: group_offsets[0] must be 0");
+    for (int g = 0; g < a->n_groups; ++g) {
+        const int32_t b = a->group_offsets[g], e = a->group_offsets[g + 1];
+        if (e <= b) return bad("contrasts: group %d is empty", g);
+        for (int32_t i = b; i < e; ++i) {
+            const int32_t c = a->group_cells[i];
+            if (c < 0 || c >= C) return bad("contrasts: group %d: cell %d outside [0, %d)", g, c, C);
+            if (i > b && c <= a->group_cells[i - 1]) return bad("contrasts: group %d: cell ids not ascending at %d", g, c);
+        }
+    }
+    p.has_batch = a->batch != nullptr && a->n_batch_levels > 1;
+    if (a->n_zero != 1 && a->n_zero != N) return bad("contrasts: n_zero must be 1 or n_genes");
+    if (!a->zero_index || (p.has_batch && !a->zero_index_adjusted))
+        return bad("contrasts: zero_index (and zero_index_adjusted with batch) are required");
+    TRY(validate_index(a->zero_index, (size_t)a->n_zero, 1, 2 * K, "zero_index"));
+    p.zi.assign(a->zero_index, a->zero_index + a->n_zero);
+    if (p.has_batch) {
+        TRY(validate_index(a->zero_index_adjusted, (size_t)a->n_zero, 1, 4 * K - 2, "zero_index_adjusted"));
+        p.zi_adj.assign(a->zero_index_adjusted, a->zero_index_adjusted + a->n_zero);
+        for (int c = 0; c < C; ++c)
+            if (a->batch[c] >= a->n_batch_levels)
+                return bad("batch[%d] = %d outside [0, %d) (negative = NA)", c, a->batch[c], a->n_batch_levels);
+    }
+    p.C = C;
+    p.K = K;
+    p.N = N;
+    p.n_zero = a->n_zero;
+    p.n_contrasts = a->n_contrasts;
+    p.n_boot = a->n_boot;
+    p.want_post = o->difference_posterior || o->adjusted_difference_posterior;
+    std::vector<int> slot_of(a->n_groups, -1);
+    p.pair_slot.resize(2 * (size_t)a->n_contrasts);
+    for (int c = 0; c < a->n_contrasts; ++c) {
+        const int ga = a->pairs[2 * c], gb = a->pairs[2 * c + 1];
+        if (ga < 0 || ga >= a->n_groups || gb < 0 || gb >= a->n_groups)
+            return bad("contrast %d names group %d outside [0, %d)", c, ga < 0 || ga >= a->n_groups ? ga : gb, a->n_groups);
+        if (ga == gb) return bad("contrast %d compares group %d with itself", c, ga);
+        // the two sides of one contrast must not share a cell (both lists are ascending)
+        int32_t i = a->group_offsets[ga], j = a->group_offsets[gb];
+        while (i < a->group_offsets[ga + 1] && j < a->group_offsets[gb + 1]) {
+            const int32_t x = a->group_cells[i], y = a->group_cells[j];
+            if (x == y) return bad("contrast %d: groups %d and %d share cell %d", c, ga, gb, x);
+            if (x < y) ++i; else ++j;
+        }
+        for (int s = 0; s < 2; ++s) {
+            const int g = s ? gb : ga;
+            if (slot_of[g] < 0) {
+                slot_of[g] = (int)p.slot_group.size();
+                p.slot_group.push_back(g);
+            }
+            p.pair_slot[2 * c + s] = slot_of[g];
+        }
+    }
+    // group joints: cells of every slot, draws once per distinct group size (local indices, src/jpmatLogBoot.cpp:221,254-257)
+    std::map<int, int64_t> draws_of_size;
+    p.cell_off.assign(1, 0);
+    for (int g : p.slot_group) {
+        const int32_t b = a->group_offsets[g], e = a->group_offsets[g + 1];
+        p.cells.insert(p.cells.end(), a->group_cells + b, a->group_cells + e);
+        p.cell_off.push_back((int64_t)p.cells.size());
+        const int n = e - b;
+        auto it = draws_of_size.find(n);
+        if (it == draws_of_size.end()) {
+            it = draws_of_size.emplace(n, (int64_t)p.draws.size()).first;
+            const std::vector<int32_t> d = gen_boot(a->seed, n, a->n_boot);
+            p.draws.insert(p.draws.end(), d.begin(), d.end());
+        }
+        p.draw_off.push_back(it->second);
+    }
+    if (!p.has_batch) return SCDE_B200_OK;
+    // batch joints: one per distinct composition table(batch[group]) (R/functions.R:355-357), pools over all cells with a
+    // non-NA batch (tapply(seq_len(n) - 1, batch, I), :570)
+    const int L = a->n_batch_levels;
+    std::vector<int32_t> off(L + 1, 0), pool;
+    for (int c = 0; c < C; ++c)
+        if (a->batch[c] >= 0) off[a->batch[c] + 1]++;
+    for (int l = 0; l < L; ++l) off[l + 1] += off[l];
+    pool.resize(off[L] > 0 ? off[L] : 1);
+    {
+        std::vector<int32_t> pos(off.begin(), off.end() - 1);
+        for (int c = 0; c < C; ++c)
+            if (a->batch[c] >= 0) pool[pos[a->batch[c]]++] = c;
+    }
+    std::map<std::vector<int32_t>, int> bslot_of;
+    std::vector<int> bslot_of_slot(p.slot_group.size());
+    for (size_t s = 0; s < p.slot_group.size(); ++s) {
+        std::vector<int32_t> comp(L, 0);
+        int D = 0;
+        for (int64_t i = p.cell_off[s]; i < p.cell_off[s + 1]; ++i)
+            if (a->batch[p.cells[i]] >= 0) {
+                comp[a->batch[p.cells[i]]]++;
+                ++D;
+            }
+        auto it = bslot_of.find(comp);
+        if (it == bslot_of.end()) {
+            it = bslot_of.emplace(comp, (int)p.bslot_D.size()).first;
+            p.bslot_D.push_back(D);
+            p.bdraw_off.push_back((int64_t)p.bdraws.size());
+            p.bdraws.resize(p.bdraws.size() + (size_t)a->n_boot * D);
+            TRY(scde_b200_batch_boot_indices(a->seed, L, off.data(), pool.data(), comp.data(), a->n_boot,
+                                             p.bdraws.data() + p.bdraw_off.back()));
+        }
+        bslot_of_slot[s] = it->second;
+    }
+    p.pair_bslot.resize(p.pair_slot.size());
+    for (size_t i = 0; i < p.pair_slot.size(); ++i) p.pair_bslot[i] = bslot_of_slot[p.pair_slot[i]];
+    if (a->batch_models) {
+        p.batch_models = a->batch_models;
+        p.b_local_theta = a->batch_local_theta;
+        p.b_sqlogit = a->batch_square_logit_conc;
+        p.b_fast_theta = !a->batch_local_theta && theta_all_regular(a->batch_models, C, C);
+    }
+    return SCDE_B200_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int scde_b200_dataset_create(scde_b200_ctx *ctx, const scde_b200_dataset_args *a, scde_b200_dataset **out,
+                             scde_b200_stats *stats) {
+    CHECK_CTX(ctx);
+    if (!a || !out) {
+        set_error("dataset_create: null argument");
+        return SCDE_B200_EINVAL;
+    }
+    *out = nullptr;
+    if (!a->counts || !a->models || !a->prior_x || !a->prior_y || a->n_genes < 1 || a->n_cells < 1 || a->n_grid < 2) {
+        set_error("dataset_create: bad arguments");
+        return SCDE_B200_EINVAL;
+    }
+    const std::vector<scde_b200_ctx *> devs = context_devices(ctx);
+    for (auto *d : devs)
+        if (d->ws_busy) {
+            set_error("another expression_difference job is alive on this context (free it first)");
+            return SCDE_B200_EINVAL;
+        }
+    const int n = (int)devs.size() < a->n_genes ? (int)devs.size() : a->n_genes;
+    scde_b200_dataset *ds = new scde_b200_dataset();
+    ds->owner = ctx;
+    ds->n_genes = a->n_genes;
+    ds->n_cells = a->n_cells;
+    ds->n_grid = a->n_grid;
+    ds->shards.assign(n, nullptr);
+    std::vector<scde_b200_stats> sst(n);
+    const int r = on_shards(n, devs, [&](int i) -> int {
+        int b = 0, e = 0;
+        shard_range(a->n_genes, n, i, &b, &e);
+        TRY(shard_create(devs[i], a, b, e, &ds->shards[i]));
+        ds->shards[i]->timer.collect(&sst[i]);
+        sst[i].table_rows = ds->shards[i]->ws->table.n_rows;
+        return SCDE_B200_OK;
+    }, &sst, stats);
+    if (r != SCDE_B200_OK) {
+        for (auto *&s : ds->shards) {
+            delete s;
+            s = nullptr;
+        }
+        delete ds;
+        cudaSetDevice(ctx->device);
+        return r;
+    }
+    *out = ds;
+    return SCDE_B200_OK;
+}
+
+int scde_b200_dataset_contrasts(scde_b200_ctx *ctx, scde_b200_dataset *ds, const scde_b200_contrast_args *a,
+                                const scde_b200_contrast_out *o, scde_b200_stats *stats) {
+    CHECK_CTX(ctx);
+    if (!ds || !a || !o) {
+        set_error("dataset_contrasts: null argument");
+        return SCDE_B200_EINVAL;
+    }
+    if (ds->owner != ctx) {
+        set_error("dataset_contrasts: the dataset belongs to another context");
+        return SCDE_B200_EINVAL;
+    }
+    ContrastPlan p;
+    try {
+        TRY(plan_contrasts(ds, a, o, p));
+    } catch (const std::bad_alloc &) {
+        set_error("dataset_contrasts: host allocation failed");
+        return SCDE_B200_ENOMEM;
+    }
+    const std::vector<scde_b200_ctx *> devs = context_devices(ctx);
+    const int n = (int)ds->shards.size();
+    std::vector<scde_b200_stats> sst(n);
+    TRY(on_shards(n, devs, [&](int i) -> int { return shard_contrasts(*ds->shards[i], p, o, &sst[i]); }, &sst, stats));
+    // Benjamini-Hochberg per contrast over all genes, on the host, once every shard has landed
+    const int N = ds->n_genes;
+    for (int c = 0; c < a->n_contrasts; ++c) {
+        const size_t off = (size_t)c * N;
+        if (o->cz) scde::bh_cz(o->z + off, N, o->cz + off);
+        if (p.has_batch && o->batch_cz) scde::bh_cz(o->batch_z + off, N, o->batch_cz + off);
+        if (p.has_batch && o->adjusted_cz) scde::bh_cz(o->adjusted_z + off, N, o->adjusted_cz + off);
+    }
+    return SCDE_B200_OK;
+}
+
+void scde_b200_dataset_free(scde_b200_ctx *ctx, scde_b200_dataset *ds) {
+    delete ds;  // every shard releases its context's workspace
+    if (ctx) cudaSetDevice(ctx->device);
 }
 
 }  // extern "C"

@@ -231,6 +231,12 @@ cudaError_t launch_softmax_i8(const ContractI8Args &a, int g0, int n_pos, int pa
 cudaError_t launch_finalize_t(const ContractI8Args &a, int n_pos, double *t_scratch, const uint32_t *sr, cudaStream_t st);
 
 // ---- ratio_summary.cu ----------------------------------------------------------------------------
+struct RatioContrast {  // one contrast of a batched launch: its joints and its outputs (layouts as in RatioArgs)
+    const double *p1, *p2;
+    int32_t *idx;
+    double *z;
+    double *post;
+};
 struct RatioArgs {
     const double *p1, *p2;  // [n_genes][ld] row-major (gene-major) device matrices
     int ld;
@@ -243,6 +249,10 @@ struct RatioArgs {
     double *post;     // optional [n_genes][ld_post] gene-major normalised posterior
     int ld_post;
     double *raw;      // optional [n_genes][ld_post] un-normalised sliding product (matSlideMult)
+    // optional device table [n_contrasts]: one launch over (genes x contrasts), each contrast's p1, p2, idx, z and post
+    // replacing the ones above (which are then unused); every entry must have the same outputs present
+    const RatioContrast *contrasts;
+    int n_contrasts;
 };
 cudaError_t launch_ratio_summary(const RatioArgs &a, cudaStream_t st);
 cudaError_t launch_magnitude(const int32_t *counts, int64_t n, int G, const double *corr_b, const double *corr_a,

@@ -5,7 +5,7 @@
 //   quick.distribution.summary R/functions.R:5039-5053  (argmax, 2.5% / 97.5% cumulative bounds)
 //   get.ratio.posterior.Z.score R/functions.R:3514-3531 (+1e-15, renormalise, tail mass -> qnorm)
 //
-// One CTA per gene: both weighted posteriors sit in shared memory, every thread owns a few lags of the sliding
+// One CTA per gene (and contrast, in a batched launch): both weighted posteriors sit in shared memory, every thread owns a few lags of the sliding
 // product and sums them in ascending j with separately rounded multiply and add (so the 2n-1 raw values are
 // bit-identical to the reference's loop on a CPU build without FMA contraction); the row never returns to HBM
 // unless the caller asked for the posterior.  R accumulates rowSums / cumsum in 80-bit long double; the device
@@ -117,6 +117,18 @@ __global__ void __launch_bounds__(R_THREADS) ratio_summary_kernel(const RatioArg
     __shared__ double s_chunk_hi[R_THREADS / 32], s_chunk_lo[R_THREADS / 32];
     const int64_t g = blockIdx.x;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    // batched launch: blockIdx.y is the contrast, whose inputs and outputs come from the device table
+    const double *p1 = a.p1, *p2 = a.p2;
+    int32_t *idx = a.idx;
+    double *zo = a.z, *post = a.post;
+    if (a.contrasts) {
+        const RatioContrast c = a.contrasts[blockIdx.y];
+        p1 = c.p1;
+        p2 = c.p2;
+        idx = c.idx;
+        zo = c.z;
+        post = c.post;
+    }
 
     // Staging.  The sliding product below gives FOUR ADJACENT lags to a thread, so that a loaded p1[j] serves four
     // products and the four p2 values it meets are a window sliding along p2 (one new load per j): two shared-memory
@@ -131,7 +143,7 @@ __global__ void __launch_bounds__(R_THREADS) ratio_summary_kernel(const RatioArg
     for (int i = tid; i < 4 * M1 + 4 * M2; i += R_THREADS) sm[i] = 0.0;
     __syncthreads();
     for (int j = tid; j < n; j += R_THREADS) {
-        double x = a.p1[g * a.ld + j], y = a.p2[g * a.ld + j];
+        double x = p1[g * a.ld + j], y = p2[g * a.ld + j];
         if (a.prior) {
             const double w = a.prior[j];
             x = __dmul_rn(x, w);
@@ -189,7 +201,7 @@ __global__ void __launch_bounds__(R_THREADS) ratio_summary_kernel(const RatioArg
         }
     }
     __syncthreads();
-    if (!a.idx && !a.z && !a.post) return;
+    if (!idx && !zo && !post) return;
 
     // x / rowSums(x)
     dd part = {0.0, 0.0};
@@ -199,7 +211,7 @@ __global__ void __launch_bounds__(R_THREADS) ratio_summary_kernel(const RatioArg
     for (int L = tid; L < nout; L += R_THREADS) {
         double r = out[L] / rs;
         out[L] = r;
-        if (a.post) a.post[g * a.ld_post + L] = r;
+        if (post) post[g * a.ld_post + L] = r;
     }
     __syncthreads();
 
@@ -287,16 +299,16 @@ __global__ void __launch_bounds__(R_THREADS) ratio_summary_kernel(const RatioArg
         }
         const int lb1 = max(1, s_cnt[0]);           // 1-based
         const int ub1 = min(nout, s_cnt[1] + 1);    // first index with cs > 0.975, else nout
-        if (a.idx) {
-            a.idx[0 * (int64_t)a.n_genes + g] = lb1 - 1;
-            a.idx[1 * (int64_t)a.n_genes + g] = bi;
-            a.idx[2 * (int64_t)a.n_genes + g] = ub1 - 1;
+        if (idx) {
+            idx[0 * (int64_t)a.n_genes + g] = lb1 - 1;
+            idx[1 * (int64_t)a.n_genes + g] = bi;
+            idx[2 * (int64_t)a.n_genes + g] = ub1 - 1;
         }
-        if (a.z) {
+        if (zo) {
             const double zv = (out[zi - 1] + 1e-15) / rs2;
             const double zl = fmin(0.0, d_qnorm_upper(gs));
             const double zg = fmax(0.0, d_qnorm_upper(gs + zv));
-            a.z[g] = (fabs(zl) > fabs(zg)) ? zl : zg;
+            zo[g] = (fabs(zl) > fabs(zg)) ? zl : zg;
         }
     }
 }
@@ -319,8 +331,19 @@ cudaError_t launch_ratio_summary(const RatioArgs &a, cudaStream_t st) {
         cudaError_t e = cudaFuncSetAttribute(ratio_summary_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
     }
-    ratio_summary_kernel<<<a.n_genes, R_THREADS, smem, st>>>(a);
-    return cudaGetLastError();
+    if (!a.contrasts) {
+        ratio_summary_kernel<<<a.n_genes, R_THREADS, smem, st>>>(a);
+        return cudaGetLastError();
+    }
+    for (int c0 = 0; c0 < a.n_contrasts; c0 += 65535) {  // gridDim.y limit
+        RatioArgs b = a;
+        b.contrasts = a.contrasts + c0;
+        const int nc = a.n_contrasts - c0 < 65535 ? a.n_contrasts - c0 : 65535;
+        ratio_summary_kernel<<<dim3((unsigned)a.n_genes, (unsigned)nc), R_THREADS, smem, st>>>(b);
+        cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
 }
 
 cudaError_t launch_magnitude(const int32_t *counts, int64_t n, int G, const double *corr_b, const double *corr_a,
