@@ -474,6 +474,57 @@ class DifferenceJob:
             pass
 
 
+def _batch_model_matrix(models: pd.DataFrame, batch_models):
+    """batch.models (R/functions.R:304,356), the error models of the composition-sampled joints, as the column-major
+    matrix of the cells of `models` in their order: ``(matrix, local_theta, sqlogit)``, or ``(None, 0, 0)`` when they
+    are `models` themselves or not given."""
+    if batch_models is None or batch_models is models:
+        return None, 0, 0
+    if list(batch_models.index) != list(models.index):
+        if not all(c in batch_models.index for c in models.index):
+            _stop("batch.models does not cover all of the cells specified in the model matrix")
+        batch_models = batch_models.loc[list(models.index)]
+    return pack_models(batch_models)
+
+
+def _zero_indices(x: np.ndarray, expectation, G: int):
+    """The fold-change grid of the prior's grid `x`, the grid of the batch-adjusted difference, and the 1-based H0 index
+    of `expectation` in each: ``diffv, zi, adiffv, zia``."""
+    diffv = fold_change_grid(x)
+    zi = _zero_index(diffv, expectation)
+    if len(zi) not in (1, G):
+        _stop("the expectation parameter must be either one number or a vector equal to the number of genes being tested")
+    adiffv = fold_change_grid(diffv)
+    return diffv, zi, adiffv, _zero_index(adiffv, expectation)
+
+
+def _difference_result(r: dict, genes, diffv, adiffv, kcols, names, correct_batch: bool, return_posteriors: bool,
+                       stats: dict):
+    """What scde.expression.difference returns, from one contrast's arrays `r` (keys as from _diff_out; the two joint
+    posteriors under ``joint_posteriors``, labelled `names`): the ``lb mle ub ce Z cZ`` frame with ``attrs["stats"]``,
+    or the reference's list as a dict with batch correction and/or posteriors."""
+    res = _summary_frame(r["idx"], r["z"], diffv, genes, cz=r.get("cz"))
+    if not correct_batch and not return_posteriors:
+        res.attrs["stats"] = stats
+        return res
+    out = {}
+    if correct_batch:
+        out["batch.adjusted"] = _summary_frame(r["adjusted_idx"], r["adjusted_z"], adiffv, genes, cz=r.get("adjusted_cz"))
+    out["results"] = res
+    if correct_batch:
+        out["batch.effect"] = _summary_frame(r["batch_idx"], r["batch_z"], diffv, genes, cz=r.get("batch_cz"))
+    if return_posteriors:
+        out["difference.posterior"] = pd.DataFrame(r["difference_posterior"], index=genes,
+                                                   columns=["%.15g" % v for v in diffv])
+        out["joint.posteriors"] = {n: pd.DataFrame(jp, index=genes, columns=kcols)
+                                   for n, jp in zip(names, r["joint_posteriors"])}
+        if correct_batch:
+            out["batch.adjusted.difference.posterior"] = pd.DataFrame(
+                r["adjusted_difference_posterior"], index=genes, columns=["%.15g" % v for v in adiffv])
+    out["stats"] = stats
+    return out
+
+
 def scde_expression_difference(models: pd.DataFrame, counts, prior, groups=None, batch=None,
                                n_randomizations: int = 150, n_cores: int = 10, batch_models=None,
                                return_posteriors: bool = False, expectation=0, verbose: int = 0, seed: int = 1,
@@ -501,14 +552,7 @@ def scde_expression_difference(models: pd.DataFrame, counts, prior, groups=None,
             correct_batch = True
         elif verbose:
             sys.stdout.write("WARNING: only one batch level detected. Nothing to correct for.")
-    bmm, blt, bsq = None, 0, 0
-    if correct_batch and batch_models is not None and batch_models is not models:
-        # batch.models (R/functions.R:304,356): the error models of the composition-sampled joints, same cells as `models`
-        if list(batch_models.index) != list(models.index):
-            if not all(c in batch_models.index for c in models.index):
-                _stop("batch.models does not cover all of the cells specified in the model matrix")
-            batch_models = batch_models.loc[list(models.index)]
-        bmm, blt, bsq = pack_models(batch_models)
+    bmm, blt, bsq = _batch_model_matrix(models, batch_models) if correct_batch else (None, 0, 0)
     if correct_batch:
         # check batch-group interactions (R/functions.R:336-349): table(groups, batch), fisher.test, warning below 1e-3
         bgti = pd.crosstab(pd.Series(np.asarray(gcodes), name="groups"), pd.Series(np.asarray(bcodes), name="batch"))
@@ -525,13 +569,7 @@ def scde_expression_difference(models: pd.DataFrame, counts, prior, groups=None,
         sys.stdout.write(str(pd.Series([glev[c] for c in gcodes if c >= 0]).value_counts().sort_index()) + "\n")
     mm, lt, sq = pack_models(models)
     x = np.asarray(prior["x"], dtype=np.float64)
-    diffv = fold_change_grid(x)
-    zi = _zero_index(diffv, expectation)
-    G = cm.shape[0]
-    if len(zi) not in (1, G):
-        _stop("the expectation parameter must be either one number or a vector equal to the number of genes being tested")
-    adiffv = r_as_character_numeric(r_seq_length(diffv[0] - diffv[-1], diffv[-1] - diffv[0], 2 * len(diffv) - 1))
-    zia = _zero_index(adiffv, expectation)
+    diffv, zi, adiffv, zia = _zero_indices(x, expectation, cm.shape[0])
     ctx = context or _lib.default_context()
     if verbose:
         sys.stdout.write("calculating difference posterior\n")
@@ -543,34 +581,9 @@ def scde_expression_difference(models: pd.DataFrame, counts, prior, groups=None,
                                      batch_sqlogit=bsq)
     if verbose:
         sys.stdout.write("summarizing differences\n")
-    bdiffp_rep = _summary_frame(res["idx"], res["z"], diffv, genes, cz=res.get("cz"))
     with np.errstate(over="ignore"):
         kcols = ["%.15g" % v for v in np.exp(marginals_from_prior(prior))]
-
-    def _posts():
-        d = {"difference.posterior": pd.DataFrame(res["difference_posterior"], index=genes,
-                                                  columns=["%.15g" % v for v in diffv]),
-             "joint.posteriors": {glev[i]: pd.DataFrame(res["joint_posteriors"][i], index=genes, columns=kcols)
-                                  for i in range(2)}}
-        return d
-
-    if correct_batch:
-        out = {"batch.adjusted": _summary_frame(res["adjusted_idx"], res["adjusted_z"], adiffv, genes, cz=res.get("adjusted_cz")),
-               "results": bdiffp_rep,
-               "batch.effect": _summary_frame(res["batch_idx"], res["batch_z"], diffv, genes, cz=res.get("batch_cz"))}
-        if return_posteriors:
-            out.update(_posts())
-            out["batch.adjusted.difference.posterior"] = pd.DataFrame(
-                res["adjusted_difference_posterior"], index=genes, columns=["%.15g" % v for v in adiffv])
-        out["stats"] = res["stats"]
-        return out
-    if return_posteriors:
-        out = {"results": bdiffp_rep}
-        out.update(_posts())
-        out["stats"] = res["stats"]
-        return out
-    bdiffp_rep.attrs["stats"] = res["stats"]
-    return bdiffp_rep
+    return _difference_result(res, genes, diffv, adiffv, kcols, glev, correct_batch, return_posteriors, res["stats"])
 
 
 def scde_test_gene_expression_difference(gene, models: pd.DataFrame, counts: pd.DataFrame, prior, groups=None, batch=None,
@@ -739,13 +752,7 @@ class DifferenceSession:
         if batch is not None:
             bcodes, blev = _named_factor(batch, self.models.index)
             correct_batch = len(blev) > 1
-        bmm, blt, bsq = None, 0, 0
-        if correct_batch and batch_models is not None and batch_models is not self.models:
-            if list(batch_models.index) != list(self.models.index):
-                if not all(c in batch_models.index for c in self.models.index):
-                    _stop("batch.models does not cover all of the cells specified in the model matrix")
-                batch_models = batch_models.loc[list(self.models.index)]
-            bmm, blt, bsq = pack_models(batch_models)
+        bmm, blt, bsq = _batch_model_matrix(self.models, batch_models) if correct_batch else (None, 0, 0)
         if correct_batch:  # the warning of R/functions.R:336-349, per contrast
             for label, la, lb, _na, _nb in plan:
                 ia, ib = (sides[side_id[tuple(sorted(code_of[v] for v in lv))]] for lv in (la, lb))
@@ -755,12 +762,7 @@ class DifferenceSession:
                     sys.stdout.write(f"WARNING: strong interaction between groups and batches in {label}! "
                                      "Correction may be ineffective:\n")
                     sys.stdout.write(f"Fisher's Exact Test for Count Data: p-value = {pval:.4g}\n")
-        diffv = fold_change_grid(self._x)
-        zi = _zero_index(diffv, expectation)
-        if len(zi) not in (1, self.G):
-            _stop("the expectation parameter must be either one number or a vector equal to the number of genes being tested")
-        adiffv = r_as_character_numeric(r_seq_length(diffv[0] - diffv[-1], diffv[-1] - diffv[0], 2 * len(diffv) - 1))
-        zia = _zero_index(adiffv, expectation)
+        diffv, zi, adiffv, zia = _zero_indices(self._x, expectation, self.G)
         nc, ng, G, K = len(plan), len(sides), self.G, self.K
         off = np.zeros(ng + 1, dtype=np.int32)
         off[1:] = np.cumsum([len(s) for s in sides])
@@ -786,44 +788,22 @@ class DifferenceSession:
                 setattr(o, k + "_z", p_f64(r[k + "_z"]))
                 setattr(o, k + "_cz", p_f64(r[k + "_cz"]))
         if return_posteriors:
-            r["post"] = np.empty((nc, 2 * K - 1, G))
+            r["difference_posterior"] = np.empty((nc, 2 * K - 1, G))
             r["jp"] = np.empty((ng, K, G))
-            o.difference_posterior, o.joint_posteriors = p_f64(r["post"]), p_f64(r["jp"])
+            o.difference_posterior, o.joint_posteriors = p_f64(r["difference_posterior"]), p_f64(r["jp"])
             if correct_batch:
-                r["apost"] = np.empty((nc, 4 * K - 3, G))
-                o.adjusted_difference_posterior = p_f64(r["apost"])
+                r["adjusted_difference_posterior"] = np.empty((nc, 4 * K - 3, G))
+                o.adjusted_difference_posterior = p_f64(r["adjusted_difference_posterior"])
         st = _lib.Stats()
         check(lib().scde_b200_dataset_contrasts(self.ctx.handle, self._ds, C.byref(a), C.byref(o), C.byref(st)))
         self.last_stats = st.as_dict()
-        genes = self.genes
         out = {}
-        for c, (label, la, lb, na, nb) in enumerate(plan):
-            res = _summary_frame(r["idx"][c].T, r["z"][c], diffv, genes, cz=r["cz"][c])
-            posts = {}
+        for c, (label, _la, _lb, na, nb) in enumerate(plan):
+            rc = {k: (v[c].T if v.ndim == 3 else v[c]) for k, v in r.items() if k != "jp"}
             if return_posteriors:
-                ja, jb = pairs[2 * c], pairs[2 * c + 1]
-                posts = {"difference.posterior": pd.DataFrame(r["post"][c].T, index=genes, columns=["%.15g" % v for v in diffv]),
-                         "joint.posteriors": {na: pd.DataFrame(r["jp"][ja].T, index=genes, columns=self._kcols),
-                                              nb: pd.DataFrame(r["jp"][jb].T, index=genes, columns=self._kcols)}}
-            if correct_batch:
-                d = {"batch.adjusted": _summary_frame(r["adjusted_idx"][c].T, r["adjusted_z"][c], adiffv, genes,
-                                                      cz=r["adjusted_cz"][c]),
-                     "results": res,
-                     "batch.effect": _summary_frame(r["batch_idx"][c].T, r["batch_z"][c], diffv, genes, cz=r["batch_cz"][c])}
-                if return_posteriors:
-                    d.update(posts)
-                    d["batch.adjusted.difference.posterior"] = pd.DataFrame(
-                        r["apost"][c].T, index=genes, columns=["%.15g" % v for v in adiffv])
-                d["stats"] = self.last_stats
-                out[label] = d
-            elif return_posteriors:
-                d = {"results": res}
-                d.update(posts)
-                d["stats"] = self.last_stats
-                out[label] = d
-            else:
-                res.attrs["stats"] = self.last_stats
-                out[label] = res
+                rc["joint_posteriors"] = [r["jp"][pairs[2 * c]].T, r["jp"][pairs[2 * c + 1]].T]
+            out[label] = _difference_result(rc, self.genes, diffv, adiffv, self._kcols, (na, nb), correct_batch,
+                                            return_posteriors, self.last_stats)
         return out
 
     def close(self):

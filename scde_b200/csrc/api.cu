@@ -641,6 +641,268 @@ int validate_index(const int32_t *v, size_t n, int lo, int hi, const char *what)
     return SCDE_B200_OK;
 }
 
+// For its lifetime, the context contracts on the tiled FP64 (DMMA) kernel: the rerun of work the tcgen05 kernel flagged
+struct Fp64Rerun {
+    scde_b200_ctx *ctx;
+    int keep;
+    explicit Fp64Rerun(scde_b200_ctx *c) : ctx(c), keep(c->opt.contract_kernel) { ctx->opt.contract_kernel = 2; }
+    ~Fp64Rerun() { ctx->opt.contract_kernel = keep; }
+    Fp64Rerun(const Fp64Rerun &) = delete;
+    Fp64Rerun &operator=(const Fp64Rerun &) = delete;
+};
+
+// magnitudes of the prior's grid, log(max(10^x - 1, 0)) (R/functions.R:575-577)
+std::vector<double> grid_magnitudes(const double *prior_x, int K) {
+    std::vector<double> mag(K);
+    for (int k = 0; k < K; ++k) {
+        double m = std::pow(10.0, prior_x[k]) - 1;
+        if (m < 0) m = 0;
+        mag[k] = std::log(m);
+    }
+    return mag;
+}
+
+// The cells of every batch level, the pools the composition-sampled draws come from: tapply(seq_len(n) - 1, batch, I)
+// (R/functions.R:570), level l's cells ascending in pool[off[l], off[l + 1]).  batch[c] < 0 = NA: the reference drops such
+// a cell from every pool, as table(batch[ii]) (:356) drops it from the composition.
+struct BatchPools {
+    std::vector<int32_t> off, pool;
+};
+
+int batch_pools(const int32_t *batch, int C, int L, BatchPools &bp) {
+    bp.off.assign(L + 1, 0);
+    for (int c = 0; c < C; ++c) {
+        if (batch[c] >= L) {
+            set_error("batch[%d] = %d outside [0, %d) (negative = NA)", c, batch[c], L);
+            return SCDE_B200_EINVAL;
+        }
+        if (batch[c] >= 0) bp.off[batch[c] + 1]++;
+    }
+    for (int l = 0; l < L; ++l) bp.off[l + 1] += bp.off[l];
+    bp.pool.resize(bp.off[L] > 0 ? bp.off[L] : 1);  // (never NULL: scde_b200_batch_boot_indices checks its pointers)
+    std::vector<int32_t> pos(bp.off.begin(), bp.off.end() - 1);
+    for (int c = 0; c < C; ++c)
+        if (batch[c] >= 0) bp.pool[pos[batch[c]]++] = c;
+    return SCDE_B200_OK;
+}
+
+// table(batch[cells]) over L levels; returns D, the number of cells with a non-NA batch (draws per randomization)
+int batch_composition(const int32_t *batch, int L, const int32_t *cells, size_t n, std::vector<int32_t> &comp) {
+    comp.assign(L, 0);
+    int D = 0;
+    for (size_t i = 0; i < n; ++i)
+        if (batch[cells[i]] >= 0) {
+            comp[batch[cells[i]]]++;
+            ++D;
+        }
+    return D;
+}
+
+// the entries of a zero_index with n_zero = 1 or one entry per gene that genes [g0, g0 + G) use
+std::vector<int32_t> zero_slice(const int32_t *zero_index, int n_zero, int g0, int G) {
+    std::vector<int32_t> zi(n_zero == 1 ? 1 : G);
+    for (size_t i = 0; i < zi.size(); ++i) zi[i] = zero_index[n_zero == 1 ? 0 : g0 + i];
+    return zi;
+}
+
+// One set of per-cell error models on the device (C x 12, column-major) and what building table rows from it needs
+struct ModelSet {
+    DBuf<double> m;
+    int C = 0, local_theta = 0, sqlogit = 0;
+    bool fast_theta = false;  // every corr.theta finite and > 0, no local-theta fit
+};
+
+int upload_models(ModelSet &s, const double *models, int C, int local_theta, int sqlogit, cudaStream_t st) {
+    s.C = C;
+    s.local_theta = local_theta;
+    s.sqlogit = sqlogit;
+    s.fast_theta = !local_theta && theta_all_regular(models, C, C);
+    return upload(s.m, models, (size_t)C * 12, st);
+}
+
+// the table rows from the model set ms (index and row ids must be in place)
+int fill_rows(scde_b200_ctx *ctx, LpTable &t, const ModelSet &ms, const double *mag_dev, StageTimer *tm) {
+    t.fast_theta = ms.fast_theta;
+    return fill_table(ctx, t, ms.m.p, ms.C, mag_dev, ms.local_theta, ms.sqlogit, tm);
+}
+
+// the table of a differential-expression call over C cells and a K-point grid
+void init_table(const scde_b200_ctx *ctx, LpTable &t, int K, int C, bool fast_theta) {
+    t.K = K;
+    t.ld = table_ld(K);
+    t.sentinel = -DBL_MAX / C / 1.1;
+    t.fast_theta = fast_theta;
+    t.zero_base = t.ld <= KP_TILED && ctx->opt.zero_base;
+    t.want_q = want_i8(ctx);
+    t.want_modes = false;
+}
+
+int workspace_busy(const scde_b200_ctx *ctx) {
+    if (!ctx->ws_busy) return SCDE_B200_OK;
+    set_error("another expression_difference job is alive on this context (free it first)");
+    return SCDE_B200_EINVAL;
+}
+
+// the context's DiffWorkspace for one job or dataset shard, held until that releases it (ctx->ws_busy = false)
+int acquire_workspace(scde_b200_ctx *ctx) {
+    TRY(workspace_busy(ctx));
+    if (!ctx->ws) ctx->ws = new DiffWorkspace();
+    ctx->ws_busy = true;
+    return SCDE_B200_OK;
+}
+
+// The three ratio passes of a difference call over G genes with their shared geometry; the caller fills in the joints and
+// outputs (RatioArgs' single-pair pointers, or a contrast table).
+struct RatioPasses {
+    RatioArgs main;      // the group joints' ratio with the prior, H0 at zero_index
+    RatioArgs batch;     // batch.effect: the batch joints' ratio, default expectation = 0 (R/functions.R:362): H0 index =
+                         // centre of the grid, handled in-kernel as index n (1-based) when zero_index is NULL
+    RatioArgs adjusted;  // batch adjustment: the two 2K-1 posteriors slid without prior weighting (R/functions.R:391)
+};
+
+RatioPasses ratio_passes(int G, int K, int ld, const double *prior_y, const int32_t *zi, const int32_t *zi_adj, int n_zero) {
+    const int nout = 2 * K - 1;
+    RatioPasses r{};
+    r.main.ld = ld;
+    r.main.n_genes = G;
+    r.main.n = K;
+    r.main.prior = prior_y;
+    r.main.zero_index = zi;
+    r.main.n_zero = n_zero == 1 ? 1 : G;
+    r.main.ld_post = round_up(nout, 8);
+    r.batch = r.main;
+    r.batch.zero_index = nullptr;
+    r.batch.n_zero = 1;
+    r.adjusted.ld = r.main.ld_post;
+    r.adjusted.n_genes = G;
+    r.adjusted.n = nout;
+    r.adjusted.prior = nullptr;
+    r.adjusted.zero_index = zi_adj;
+    r.adjusted.n_zero = r.main.n_zero;
+    r.adjusted.ld_post = round_up(2 * nout - 1, 8);
+    return r;
+}
+
+// the main pass, and with a batch factor the batch.effect and adjusted passes after it
+int launch_ratio_passes(const RatioPasses &r, bool has_batch, cudaStream_t st) {
+    SCDE_CUDA(launch_ratio_summary(r.main, st));
+    if (has_batch) {
+        SCDE_CUDA(launch_ratio_summary(r.batch, st));
+        SCDE_CUDA(launch_ratio_summary(r.adjusted, st));
+    }
+    return SCDE_B200_OK;
+}
+
+// Where a job's per-gene results go in the caller's (column-major) output matrices: row `row0` of matrices with `ld`
+// rows.  A single-device call writes whole matrices (ld = the job's genes, row0 = 0); the shards of a multi-device call
+// write their gene range of the same buffers.
+struct OutPlace {
+    int64_t ld, row0;
+};
+
+// a [3][G] block of grid indices and a Z vector on the device -> rows pl.row0.. of block `block` of the caller's outputs
+// (blocks of pl.ld x 3 and pl.ld); a NULL destination is skipped
+int download_summary(cudaStream_t st, int G, const int32_t *idx, const double *z, int32_t *idx_dst, double *z_dst,
+                     OutPlace pl, size_t block = 0) {
+    if (idx_dst)
+        SCDE_CUDA(cudaMemcpy2DAsync(idx_dst + block * 3 * pl.ld + pl.row0, sizeof(int32_t) * (size_t)pl.ld, idx,
+                                    sizeof(int32_t) * (size_t)G, sizeof(int32_t) * (size_t)G, 3, cudaMemcpyDeviceToHost, st));
+    if (z_dst)
+        SCDE_CUDA(cudaMemcpyAsync(z_dst + block * pl.ld + pl.row0, z, sizeof(double) * (size_t)G, cudaMemcpyDeviceToHost, st));
+    return SCDE_B200_OK;
+}
+
+// stage times and launches of the timer, the table's rows and the list entries the joints contracted (the stream has
+// drained)
+int collect_stats(StageTimer &tm, const DiffWorkspace *ws, scde_b200_stats *stats) {
+    if (!stats) return SCDE_B200_OK;
+    tm.collect(stats);
+    stats->table_rows = ws->table.n_rows;
+    unsigned long long tot = 0;
+    SCDE_CUDA(cudaMemcpy(&tot, ws->scr.total.p, sizeof(tot), cudaMemcpyDeviceToHost));
+    stats->contract_cells = (int64_t)tot;
+    return SCDE_B200_OK;
+}
+
+// Benjamini-Hochberg cZ over the n genes of result block `block` for every Z whose cZ the caller asked for
+template <class Out>
+void bh_outputs(const Out *o, bool has_batch, int n, size_t block = 0) {
+    const size_t off = block * n;
+    if (o->cz) scde::bh_cz(o->z + off, n, o->cz + off);
+    if (has_batch && o->batch_cz) scde::bh_cz(o->batch_z + off, n, o->batch_cz + off);
+    if (has_batch && o->adjusted_cz) scde::bh_cz(o->adjusted_z + off, n, o->adjusted_cz + off);
+}
+
+// shard i of n over genes [0, N): contiguous ranges, the first N % n of them one gene longer
+void shard_range(int N, int n, int i, int *b, int *e) {
+    const int base = N / n, rem = N % n;
+    *b = i * base + (i < rem ? i : rem);
+    *e = *b + base + (i < rem ? 1 : 0);
+}
+
+// Runs f(i) for i < n on one host thread each (directly when n == 1); exceptions become return codes, the first failing
+// shard's error text becomes this thread's.
+template <class F>
+int on_shards(int n, const std::vector<scde_b200_ctx *> &devs, F f, std::vector<scde_b200_stats> *sst, scde_b200_stats *stats) {
+    std::vector<int> rc(n, SCDE_B200_OK);
+    std::vector<std::string> msg(n);
+    auto body = [&](int i) {
+        try {
+            rc[i] = f(i);
+            if (rc[i] != SCDE_B200_OK) msg[i] = g_err;  // the error text is thread-local
+        } catch (const std::bad_alloc &) {
+            rc[i] = SCDE_B200_ENOMEM;
+            msg[i] = "host allocation failed";
+        } catch (const std::exception &ex) {
+            rc[i] = SCDE_B200_EINVAL;
+            msg[i] = ex.what();
+        } catch (...) {
+            rc[i] = SCDE_B200_EINVAL;
+            msg[i] = "unknown exception";
+        }
+    };
+    if (n == 1) {
+        body(0);
+    } else {
+        std::vector<std::thread> th;
+        try {
+            for (int i = 0; i < n; ++i) th.emplace_back(body, i);
+        } catch (...) {
+            for (auto &t : th) t.join();
+            set_error("could not start a host thread per device");
+            return SCDE_B200_ENOMEM;
+        }
+        for (auto &t : th) t.join();
+    }
+    cudaSetDevice(devs[0]->device);
+    for (int i = 0; i < n; ++i)
+        if (rc[i] != SCDE_B200_OK) {
+            if (n == 1)
+                g_err = msg[i];
+            else
+                set_error("device %d (shard %d of %d): %s", devs[i]->device, i, n, msg[i].c_str());
+            return rc[i];
+        }
+    if (stats && sst) {  // stage times: the slowest shard; counters: summed
+        memset(stats, 0, sizeof(*stats));
+        for (int i = 0; i < n; ++i) {
+            for (int k = 0; k < SCDE_B200_T_COUNT; ++k) {
+                if ((*sst)[i].ms[k] > stats->ms[k]) stats->ms[k] = (*sst)[i].ms[k];
+                stats->launches[k] += (*sst)[i].launches[k];
+            }
+            stats->table_rows += (*sst)[i].table_rows;
+            stats->contract_cells += (*sst)[i].contract_cells;
+        }
+    }
+    return SCDE_B200_OK;
+}
+
+std::vector<scde_b200_ctx *> context_devices(scde_b200_ctx *ctx) {
+    std::vector<scde_b200_ctx *> devs{ctx};
+    for (auto *c : ctx->children) devs.push_back(c);
+    return devs;
+}
+
 }  // namespace
 
 // ============================================================================================
@@ -947,12 +1209,10 @@ static int log_boot_common(scde_b200_ctx *ctx, const double *models, int32_t n_c
     int rerun = 0;
     TRY(read_flags(ctx, &rerun));
     if (rerun) {  // a cell drawn more than 127 times in one randomization: outside the int8 operand range
-        const int keep = ctx->opt.contract_kernel;
-        ctx->opt.contract_kernel = 2;
+        const Fp64Rerun f64(ctx);
         r = log_boot_impl(ctx, models, n_cells, ucl_flat, ucl_offsets, uci, n_genes, magnitudes, n_grid, n_boot, boot_idx, D,
                           return_individual, local_theta, square_logit_conc, ensemble, modes_flag, post_flag, jp, modes,
                           post);
-        ctx->opt.contract_kernel = keep;
     }
     return r;
 }
@@ -1433,15 +1693,14 @@ int scde_b200_probe_contract_i8(scde_b200_ctx *ctx, const int8_t *qtable, int32_
 // scde.expression.difference on the device (R/functions.R:304-408)
 struct scde_b200_diff_job {
     int G = 0, C = 0, K = 0, n_boot = 0, n_levels = 0;
-    int local_theta = 0, sqlogit = 0, want_post = 0, has_batch = 0;
+    int want_post = 0, has_batch = 0;
     int n_group[2] = {0, 0};
     int n_zero = 1;
     DiffWorkspace *ws = nullptr;
     scde_b200_ctx *owner = nullptr;
-    DBuf<double> models, mag, prior_y;
-    DBuf<double> bmodels;       // batch.models when they differ from models (else empty)
-    int b_local_theta = 0, b_sqlogit = 0;
-    bool fast_theta = false, b_fast_theta = false;
+    ModelSet models;
+    ModelSet bmodels;           // batch.models when they differ from models (else empty)
+    DBuf<double> mag, prior_y;
     DBuf<int32_t> cell_ids[2];  // group cell lists
     DBuf<int32_t> boot[4];
     int D[4] = {0, 0, 0, 0};
@@ -1449,7 +1708,6 @@ struct scde_b200_diff_job {
     DBuf<int32_t> idx, bidx, aidx;
     DBuf<double> z, bz, az;
     StageTimer timer;
-    int64_t contract_cells = 0;
     bool ran = false;
     int64_t known_rows = 0;          // table rows of the last completed run of this job (0: unknown): the next run needs no
                                      // size read-back -- same counts, same rows
@@ -1487,36 +1745,16 @@ int upload_draws(scde_b200_ctx *ctx, scde_b200_diff_job *j, const scde_b200_diff
         j->D[i] = n;
     }
     if (j->has_batch) {
-        // batch[c] < 0 = NA: the reference's tapply(seq_len(n) - 1, batch, I) (R/functions.R:570) and table(batch[ii])
-        // (:356) both drop NA entries -- such a cell is in no pool and does not count towards the composition
         const int L = a->n_batch_levels;
-        std::vector<int32_t> off(L + 1, 0), cells;
-        for (int c = 0; c < C; ++c) {
-            if (a->batch[c] >= L) {
-                set_error("batch[%d] = %d outside [0, %d) (negative = NA)", c, a->batch[c], L);
-                return SCDE_B200_EINVAL;
-            }
-            if (a->batch[c] >= 0) off[a->batch[c] + 1]++;
-        }
-        for (int l = 0; l < L; ++l) off[l + 1] += off[l];
-        cells.resize(off[L] > 0 ? off[L] : 1);  // (never NULL: scde_b200_batch_boot_indices checks its pointers)
-        {
-            std::vector<int32_t> pos(off.begin(), off.end() - 1);
-            for (int c = 0; c < C; ++c)
-                if (a->batch[c] >= 0) cells[pos[a->batch[c]]++] = c;  // tapply(0:(n-1), batch, I): ascending
-        }
+        BatchPools bp;
+        TRY(batch_pools(a->batch, C, L, bp));
         for (int i = 0; i < 2; ++i) {
-            std::vector<int32_t> comp(L, 0);  // table(batch[ii])
-            int D = 0;
-            for (int c : j->ids[i])
-                if (a->batch[c] >= 0) {
-                    comp[a->batch[c]]++;
-                    ++D;
-                }
+            std::vector<int32_t> comp;
+            const int D = batch_composition(a->batch, L, j->ids[i].data(), j->ids[i].size(), comp);
             src[2 + i] = a->boot_idx[2 + i];
             if (!src[2 + i]) {
                 j->gen[2 + i].resize((size_t)a->n_boot * D);
-                TRY(scde_b200_batch_boot_indices(a->seed, L, off.data(), cells.data(), comp.data(), a->n_boot,
+                TRY(scde_b200_batch_boot_indices(a->seed, L, bp.off.data(), bp.pool.data(), comp.data(), a->n_boot,
                                                  j->gen[2 + i].data()));
                 src[2 + i] = j->gen[2 + i].data();
             }
@@ -1637,6 +1875,18 @@ int start_count_copies(scde_b200_ctx *ctx, scde_b200_diff_job *j, const int32_t 
     return SCDE_B200_OK;
 }
 
+// the genes [g0, g1) a call processes: [gene_begin, gene_end), all of them when both are 0
+static int gene_range(const scde_b200_diff_args *a, int *g0, int *g1) {
+    *g0 = a->gene_begin;
+    *g1 = a->gene_end;
+    if (*g0 == 0 && *g1 == 0) *g1 = a->n_genes;
+    if (*g0 < 0 || *g1 > a->n_genes || *g0 >= *g1) {
+        set_error("gene range [%d, %d) invalid for %d genes", *g0, *g1, a->n_genes);
+        return SCDE_B200_EINVAL;
+    }
+    return SCDE_B200_OK;
+}
+
 // defer_counts: the count matrix is not copied here (the one-shot call overlaps its upload with the table build)
 static int diff_upload_impl(scde_b200_ctx *ctx, const scde_b200_diff_args *a, int32_t want_posteriors,
                             scde_b200_diff_job **out, bool defer_counts) {
@@ -1648,12 +1898,8 @@ static int diff_upload_impl(scde_b200_ctx *ctx, const scde_b200_diff_args *a, in
         set_error("expression_difference: bad arguments");
         return SCDE_B200_EINVAL;
     }
-    int g0 = a->gene_begin, g1 = a->gene_end;
-    if (g0 == 0 && g1 == 0) g1 = a->n_genes;
-    if (g0 < 0 || g1 > a->n_genes || g0 >= g1) {
-        set_error("gene range [%d, %d) invalid for %d genes", g0, g1, a->n_genes);
-        return SCDE_B200_EINVAL;
-    }
+    int g0 = 0, g1 = 0;
+    TRY(gene_range(a, &g0, &g1));
     const int G = g1 - g0, C = a->n_cells, K = a->n_grid;
     std::vector<int32_t> ids[2];
     for (int c = 0; c < C; ++c)
@@ -1672,15 +1918,10 @@ static int diff_upload_impl(scde_b200_ctx *ctx, const scde_b200_diff_args *a, in
         return SCDE_B200_EINVAL;
     }
     cudaStream_t st = ctx->stream;
-    if (ctx->ws_busy) {
-        set_error("another expression_difference job is alive on this context (free it first)");
-        return SCDE_B200_EINVAL;
-    }
-    if (!ctx->ws) ctx->ws = new DiffWorkspace();
+    TRY(acquire_workspace(ctx));
     scde_b200_diff_job *j = new scde_b200_diff_job();
     j->ws = ctx->ws;
     j->owner = ctx;
-    ctx->ws_busy = true;
     auto fail = [&](int r) {
         if (j->copy_chunks) cudaStreamSynchronize(ctx->copy_stream);  // the copy engine reads the caller's buffer
         ctx->ws_busy = false;
@@ -1701,8 +1942,6 @@ static int diff_upload_impl(scde_b200_ctx *ctx, const scde_b200_diff_args *a, in
     j->C = C;
     j->K = K;
     j->n_boot = a->n_boot;
-    j->local_theta = a->local_theta;
-    j->sqlogit = a->square_logit_conc;
     j->want_post = want_posteriors;
     j->has_batch = has_batch;
     j->n_levels = has_batch ? a->n_batch_levels : 0;
@@ -1722,20 +1961,11 @@ static int diff_upload_impl(scde_b200_ctx *ctx, const scde_b200_diff_args *a, in
                 std::chrono::duration<double, std::milli>(tu1 - tu0).count(), sizeof(int32_t) * (double)G * C / 1e6,
                 std::chrono::duration<double, std::milli>(tu2 - tu1).count());
     }
-    JTRY(upload(j->models, a->models, (size_t)C * 12, st));
-    if (has_batch && a->batch_models && a->batch_models != a->models) {
-        JTRY(upload(j->bmodels, a->batch_models, (size_t)C * 12, st));
-        j->b_local_theta = a->batch_local_theta;
-        j->b_sqlogit = a->batch_square_logit_conc;
-        j->b_fast_theta = !a->batch_local_theta && theta_all_regular(a->batch_models, C, C);
-    }
+    JTRY(upload_models(j->models, a->models, C, a->local_theta, a->square_logit_conc, st));
+    if (has_batch && a->batch_models && a->batch_models != a->models)
+        JTRY(upload_models(j->bmodels, a->batch_models, C, a->batch_local_theta, a->batch_square_logit_conc, st));
     JTRY(upload(j->prior_y, a->prior_y, (size_t)K, st));
-    std::vector<double> mag(K);
-    for (int k = 0; k < K; ++k) {  // R/functions.R:575-577
-        double m = std::pow(10.0, a->prior_x[k]) - 1;
-        if (m < 0) m = 0;
-        mag[k] = std::log(m);
-    }
+    const std::vector<double> mag = grid_magnitudes(a->prior_x, K);
     JTRY(upload(j->mag, mag.data(), (size_t)K, st));
     for (int i = 0; i < 2; ++i) {
         j->n_group[i] = (int)ids[i].size();
@@ -1750,14 +1980,13 @@ static int diff_upload_impl(scde_b200_ctx *ctx, const scde_b200_diff_args *a, in
     else
         JTRY(upload_draws(ctx, j, a));
     {
-        std::vector<int32_t> zi(a->n_zero == 1 ? 1 : G);
-        for (size_t i = 0; i < zi.size(); ++i) zi[i] = a->zero_index[a->n_zero == 1 ? 0 : g0 + i];
+        const std::vector<int32_t> zi = zero_slice(a->zero_index, a->n_zero, g0, G);
         JTRY(validate_index(zi.data(), zi.size(), 1, 2 * K, "zero_index"));
         JTRY(upload(j->zi, zi.data(), zi.size(), st));
         if (has_batch) {
-            for (size_t i = 0; i < zi.size(); ++i) zi[i] = a->zero_index_adjusted[a->n_zero == 1 ? 0 : g0 + i];
-            JTRY(validate_index(zi.data(), zi.size(), 1, 4 * K - 2, "zero_index_adjusted"));
-            JTRY(upload(j->zi_adj, zi.data(), zi.size(), st));
+            const std::vector<int32_t> za = zero_slice(a->zero_index_adjusted, a->n_zero, g0, G);
+            JTRY(validate_index(za.data(), za.size(), 1, 4 * K - 2, "zero_index_adjusted"));
+            JTRY(upload(j->zi_adj, za.data(), za.size(), st));
         }
         JCUDA(cudaStreamSynchronize(st));
     }
@@ -1774,13 +2003,7 @@ static int diff_upload_impl(scde_b200_ctx *ctx, const scde_b200_diff_args *a, in
         JCUDA(j->az.ensure((size_t)G));
         if (want_posteriors) JCUDA(j->ws->apost.ensure((size_t)G * lda));
     }
-    j->ws->table.K = K;
-    j->ws->table.ld = ld;
-    j->ws->table.sentinel = -DBL_MAX / C / 1.1;
-    j->fast_theta = !a->local_theta && theta_all_regular(a->models, C, C);
-    j->ws->table.fast_theta = j->fast_theta;
-    j->ws->table.zero_base = ld <= KP_TILED && ctx->opt.zero_base;
-    j->ws->table.want_q = want_i8(ctx);
+    init_table(ctx, j->ws->table, K, C, j->models.fast_theta);  // the chunked front's table plan reads models' fast_theta
     JCUDA(cudaStreamSynchronize(st));
     // last: the small uploads above share the one H2D copy engine with these 1.2 GB and would queue behind them
     if (defer_counts) JTRY(start_count_copies(ctx, j, a->counts + g0, a->n_genes));
@@ -1807,7 +2030,7 @@ static int front_chunked(scde_b200_ctx *ctx, scde_b200_diff_job *j, int phase, b
     t.n_cells = C;
     t.n_genes = G;
     t.ld_ridx = C;
-    if (phase == 0) j->front_plan = plan_table(ctx, t, j->local_theta);
+    if (phase == 0) j->front_plan = plan_table(ctx, t, j->models.local_theta);
     TablePlan &pl = j->front_plan;  // prepare_cells and reserve_rows bind its buffers in phase 0
     // the copies are already in flight (start_count_copies); every path below waits for them on the compute stream
     const bool pipelined = pl.q_fused && t.zero_base && C >= 64 * j->copy_chunks && ctx->opt.pipeline_front;
@@ -1846,7 +2069,7 @@ static int front_chunked(scde_b200_ctx *ctx, scde_b200_diff_job *j, int phase, b
         FCUDA(t.dedup_bits.ensure(dedup_scratch_words(C)));
         FCUDA(cudaMemsetAsync(t.err.p, 0, sizeof(int32_t), st));
         e0 = tm.begin(st);
-        FTRY(prepare_cells(ctx, t, pl, j->models.p, C, j->mag.p, j->local_theta, j->sqlogit));
+        FTRY(prepare_cells(ctx, t, pl, j->models.m.p, C, j->mag.p, j->models.local_theta, j->models.sqlogit));
         tm.end(SCDE_B200_T_LPTABLE, e0, st, 1);
         j->front_cap = 0;
     }
@@ -1880,7 +2103,7 @@ static int front_chunked(scde_b200_ctx *ctx, scde_b200_diff_job *j, int phase, b
         tm.end(SCDE_B200_T_DEDUP, e0, st, 5);
         e0 = tm.begin(st);
         int nl = 0;
-        FTRY(launch_table_rows(ctx, t, pl, CellRange{c0, c0 + n, cap}, j->models.p, C, j->local_theta, &nl));
+        FTRY(launch_table_rows(ctx, t, pl, CellRange{c0, c0 + n, cap}, j->models.m.p, C, j->models.local_theta, &nl));
         tm.end(SCDE_B200_T_LPTABLE, e0, st, nl);
     }
     tr_queued = since();
@@ -1943,13 +2166,11 @@ static int diff_run_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, bool chunked
     cudaStream_t st = ctx->stream;
     StageTimer &tm = j->timer;
     tm.reset();
-    j->contract_cells = 0;
     SCDE_CUDA(j->ws->scr.total.ensure(1));
     SCDE_CUDA(cudaMemsetAsync(j->ws->scr.total.p, 0, sizeof(unsigned long long), st));
     const int G = j->G, C = j->C, K = j->K;
-    const int ld = j->ws->table.ld, nout = 2 * K - 1, ldo = round_up(nout, 8), nadj = 2 * nout - 1, lda = round_up(nadj, 8);
+    const int ld = j->ws->table.ld;
     j->ws->table.want_q = want_i8(ctx);
-    j->ws->table.want_modes = false;
     TRY(reset_flags(ctx));
     int t_all = tm.begin(st);
     bool front_done = false, joint0_done = false;
@@ -1983,19 +2204,15 @@ static int diff_run_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, bool chunked
         const int64_t known = (!chunked_counts && want_i8(ctx)) ? j->known_rows : 0;
         TRY(index_from_counts(ctx, j->ws->table, j->ws->counts.p, G, 0, G, C, &tm, known));
         j->rows_unchecked = known > 0;
-        TRY(fill_table(ctx, j->ws->table, j->models.p, C, j->mag.p, j->local_theta, j->sqlogit, &tm));
+        TRY(fill_rows(ctx, j->ws->table, j->models, j->mag.p, &tm));
     }
     for (int i = 0; i < 2; ++i)
         if (!(i == 0 && joint0_done)) TRY(group_joint(i));
     // batch joints: all cells, composition-sampled draws are global cell ids (R/functions.R:355-357)
     if (j->has_batch) {
-        if (j->bmodels.p) {
-            // batch.models differ from models: the table rows are rebuilt from them (same row ids -- the counts have not
-            // changed -- so the index matrix stays); the group joints above are done with the first table
-            j->ws->table.fast_theta = j->b_fast_theta;
-            TRY(fill_table(ctx, j->ws->table, j->bmodels.p, C, j->mag.p, j->b_local_theta, j->b_sqlogit, &tm));
-            j->ws->table.fast_theta = j->fast_theta;
-        }
+        // batch.models differ from models: the table rows are rebuilt from them (same row ids -- the counts have not
+        // changed -- so the index matrix stays); the group joints above are done with the first table
+        if (j->bmodels.m.p) TRY(fill_rows(ctx, j->ws->table, j->bmodels, j->mag.p, &tm));
         // the two composition-sampled joints walk the same cells and rows with different draws: one launch of the contraction
         // kernel for both, items paired on neighbouring SMs, so the table is pulled from DRAM once for the two
         TwinJoint tw{j->boot_ptr[3], j->D[3], j->ws->jp[3].p, &j->ws->scr2};
@@ -2006,66 +2223,29 @@ static int diff_run_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, bool chunked
             TRY(run_joint(ctx, j->ws->table, nullptr, C, j->boot_ptr[3], j->n_boot, j->D[3], (double)j->n_boot,
                           j->ws->jp[3].p, ld, j->ws->scr, &tm, true));
     }
-    int e0 = tm.begin(st);
-    int nl = 0;
-    RatioArgs r{};
-    r.p1 = j->ws->jp[0].p;
-    r.p2 = j->ws->jp[1].p;
-    r.ld = ld;
-    r.n_genes = G;
-    r.n = K;
-    r.prior = j->prior_y.p;
-    r.zero_index = j->zi.p;
-    r.n_zero = j->n_zero == 1 ? 1 : G;
-    r.idx = j->idx.p;
-    r.z = j->z.p;
-    r.post = (j->want_post || j->has_batch) ? j->ws->post.p : nullptr;
-    r.ld_post = ldo;
-    SCDE_CUDA(launch_ratio_summary(r, st));
-    ++nl;
-    if (j->has_batch) {
-        static const int32_t mid_host = 0;
-        (void)mid_host;
-        // batch.effect is summarised with the default expectation = 0 (R/functions.R:362): H0 index = centre
-        RatioArgs b = r;
-        b.p1 = j->ws->jp[2].p;
-        b.p2 = j->ws->jp[3].p;
-        b.idx = j->bidx.p;
-        b.z = j->bz.p;
-        b.post = j->ws->bpost.p;
-        b.zero_index = nullptr;  // centre of the grid: handled in-kernel as index n (1-based) when NULL
-        b.n_zero = 1;
-        SCDE_CUDA(launch_ratio_summary(b, st));
-        ++nl;
-        // batch adjustment: slide the two 2K-1 posteriors without prior weighting (R/functions.R:391)
-        RatioArgs c{};
-        c.p1 = j->ws->post.p;
-        c.p2 = j->ws->bpost.p;
-        c.ld = ldo;
-        c.n_genes = G;
-        c.n = nout;
-        c.prior = nullptr;
-        c.zero_index = j->zi_adj.p;
-        c.n_zero = j->n_zero == 1 ? 1 : G;
-        c.idx = j->aidx.p;
-        c.z = j->az.p;
-        c.post = j->want_post ? j->ws->apost.p : nullptr;
-        c.ld_post = lda;
-        SCDE_CUDA(launch_ratio_summary(c, st));
-        ++nl;
-    }
-    tm.end(SCDE_B200_T_RATIO, e0, st, nl);
+    const int e0 = tm.begin(st);
+    RatioPasses r = ratio_passes(G, K, ld, j->prior_y.p, j->zi.p, j->zi_adj.p, j->n_zero);
+    r.main.p1 = j->ws->jp[0].p;
+    r.main.p2 = j->ws->jp[1].p;
+    r.main.idx = j->idx.p;
+    r.main.z = j->z.p;
+    r.main.post = (j->want_post || j->has_batch) ? j->ws->post.p : nullptr;
+    r.batch.p1 = j->ws->jp[2].p;
+    r.batch.p2 = j->ws->jp[3].p;
+    r.batch.idx = j->bidx.p;
+    r.batch.z = j->bz.p;
+    r.batch.post = j->ws->bpost.p;
+    r.adjusted.p1 = j->ws->post.p;
+    r.adjusted.p2 = j->ws->bpost.p;
+    r.adjusted.idx = j->aidx.p;
+    r.adjusted.z = j->az.p;
+    r.adjusted.post = j->want_post ? j->ws->apost.p : nullptr;
+    TRY(launch_ratio_passes(r, j->has_batch, st));
+    tm.end(SCDE_B200_T_RATIO, e0, st, j->has_batch ? 3 : 1);
     tm.end(SCDE_B200_T_TOTAL, t_all, st, 0);
     j->ran = true;
     return SCDE_B200_OK;
 }
-
-// Where a job's per-gene results go in the caller's (column-major) output matrices: row `row0` of matrices with `ld`
-// rows.  A single-device call writes whole matrices (ld = the job's genes, row0 = 0); the shards of a multi-device call
-// write their gene range of the same buffers.
-struct OutPlace {
-    int64_t ld, row0;
-};
 
 // [G][ld_src] gene-major device matrix -> rows row0.. of a column-major host matrix with pl.ld rows
 static int download_matrix(scde_b200_ctx *ctx, DiffWorkspace *ws, int G, const double *src, int ld_src, int cols, double *dst,
@@ -2108,29 +2288,18 @@ static int diff_download_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, const s
         int rerun = 0;
         TRY(read_flags(ctx, &rerun));
         if (rerun) {  // a multiplicity above 127: repeat the run on the FP64 contraction kernel
-            const int keep = ctx->opt.contract_kernel;
-            ctx->opt.contract_kernel = 2;
-            const int r = scde_b200_diff_run(ctx, j);
-            ctx->opt.contract_kernel = keep;
-            if (r != SCDE_B200_OK) return r;
+            {
+                const Fp64Rerun f64(ctx);
+                TRY(scde_b200_diff_run(ctx, j));
+            }
             SCDE_CUDA(cudaStreamSynchronize(st));
         }
     }
     if (o) {
-        auto get_idx = [&](int32_t *dst, const int32_t *src) {  // [3][G] on the device -> rows row0.. of an ld x 3 matrix
-            return cudaMemcpy2DAsync(dst + pl.row0, sizeof(int32_t) * (size_t)pl.ld, src, sizeof(int32_t) * (size_t)G,
-                                     sizeof(int32_t) * (size_t)G, 3, cudaMemcpyDeviceToHost, st);
-        };
-        auto get_z = [&](double *dst, const double *src) {
-            return cudaMemcpyAsync(dst + pl.row0, src, sizeof(double) * (size_t)G, cudaMemcpyDeviceToHost, st);
-        };
-        if (o->idx) SCDE_CUDA(get_idx(o->idx, j->idx.p));
-        if (o->z) SCDE_CUDA(get_z(o->z, j->z.p));
+        TRY(download_summary(st, G, j->idx.p, j->z.p, o->idx, o->z, pl));
         if (j->has_batch) {
-            if (o->batch_idx) SCDE_CUDA(get_idx(o->batch_idx, j->bidx.p));
-            if (o->batch_z) SCDE_CUDA(get_z(o->batch_z, j->bz.p));
-            if (o->adjusted_idx) SCDE_CUDA(get_idx(o->adjusted_idx, j->aidx.p));
-            if (o->adjusted_z) SCDE_CUDA(get_z(o->adjusted_z, j->az.p));
+            TRY(download_summary(st, G, j->bidx.p, j->bz.p, o->batch_idx, o->batch_z, pl));
+            TRY(download_summary(st, G, j->aidx.p, j->az.p, o->adjusted_idx, o->adjusted_z, pl));
         }
         SCDE_CUDA(cudaStreamSynchronize(st));
         for (int i = 0; i < 2; ++i) {
@@ -2156,14 +2325,7 @@ static int diff_download_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, const s
         }
     }
     SCDE_CUDA(cudaStreamSynchronize(st));
-    if (stats) {
-        j->timer.collect(stats);
-        stats->table_rows = j->ws->table.n_rows;
-        unsigned long long tot = 0;
-        SCDE_CUDA(cudaMemcpy(&tot, j->ws->scr.total.p, sizeof(tot), cudaMemcpyDeviceToHost));
-        stats->contract_cells = (int64_t)tot;  // list entries contracted, summed over genes and joints
-    }
-    return SCDE_B200_OK;
+    return collect_stats(j->timer, j->ws, stats);
 }
 
 extern "C" {
@@ -2182,7 +2344,7 @@ void scde_b200_diff_free(scde_b200_ctx *ctx, scde_b200_diff_job *job) {
 
 // one device: upload (chunked, overlapped), run, download into the caller's buffers at `pl`
 static int expression_difference_single(scde_b200_ctx *ctx, const scde_b200_diff_args *args, const scde_b200_diff_out *out,
-                                        scde_b200_stats *stats, const OutPlace *place) {
+                                        scde_b200_stats *stats, OutPlace pl) {
     CHECK_CTX(ctx);
     const int want_post = out->difference_posterior || out->adjusted_difference_posterior;
     const bool trace = ctx->opt.trace != 0;  // host wall-clock of the three phases on stderr
@@ -2198,68 +2360,13 @@ static int expression_difference_single(scde_b200_ctx *ctx, const scde_b200_diff
     r = diff_run_impl(ctx, job, true);
     if (r != SCDE_B200_OK && ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);
     const auto t2 = now();
-    if (r == SCDE_B200_OK) r = diff_download_impl(ctx, job, out, stats, place ? *place : OutPlace{job->G, 0});
+    if (r == SCDE_B200_OK) r = diff_download_impl(ctx, job, out, stats, pl);
     const auto t3 = now();
     scde_b200_diff_free(ctx, job);
     if (trace)
         fprintf(stderr, "[scde_b200] expression_difference (device %d): upload %.2f ms, run (queued) %.2f ms, download (incl. wait) %.2f ms, free %.2f ms\n",
                 ctx->device, ms(t0, t1), ms(t1, t2), ms(t2, t3), ms(t3, now()));
     return r;
-}
-
-// Several devices: contiguous gene ranges, one per device (the split the reference's chunk() makes for n.cores,
-// R/functions.R:606), one host thread per device, every shard with the same Seed and therefore the same draws -- the
-// n.cores = 1 semantics, so the result does not depend on the number of devices.  No inter-GPU traffic: every shard's
-// results go to its rows of the caller's buffers by device-to-host copies (north_star: "or by a host copy").
-static int expression_difference_multi(scde_b200_ctx *ctx, const scde_b200_diff_args *args, const scde_b200_diff_out *out,
-                                       scde_b200_stats *stats) {
-    int g0 = args->gene_begin, g1 = args->gene_end;
-    if (g0 == 0 && g1 == 0) g1 = args->n_genes;
-    if (g0 < 0 || g1 > args->n_genes || g0 >= g1) {
-        set_error("gene range [%d, %d) invalid for %d genes", g0, g1, args->n_genes);
-        return SCDE_B200_EINVAL;
-    }
-    std::vector<scde_b200_ctx *> devs;
-    devs.push_back(ctx);
-    for (auto *c : ctx->children) devs.push_back(c);
-    const int n = g1 - g0;
-    const int n_use = (int)devs.size() < n ? (int)devs.size() : n;
-    std::vector<int> rc(n_use, SCDE_B200_OK);
-    std::vector<std::string> msg(n_use);
-    std::vector<scde_b200_stats> sst(n_use);
-    std::vector<std::thread> th;
-    const int base = n / n_use, rem = n % n_use;
-    for (int i = 0; i < n_use; ++i) {
-        const int b = g0 + i * base + (i < rem ? i : rem), e = b + base + (i < rem ? 1 : 0);
-        th.emplace_back([&, i, b, e] {
-            scde_b200_diff_args a = *args;
-            a.gene_begin = b;
-            a.gene_end = e;
-            const OutPlace pl{n, b - g0};
-            memset(&sst[i], 0, sizeof(scde_b200_stats));
-            rc[i] = expression_difference_single(devs[i], &a, out, &sst[i], &pl);
-            if (rc[i] != SCDE_B200_OK) msg[i] = g_err;  // the error text is thread-local
-        });
-    }
-    for (auto &t : th) t.join();
-    cudaSetDevice(ctx->device);
-    for (int i = 0; i < n_use; ++i)
-        if (rc[i] != SCDE_B200_OK) {
-            set_error("device %d (shard %d of %d): %s", devs[i]->device, i, n_use, msg[i].c_str());
-            return rc[i];
-        }
-    if (stats) {  // stage times: the slowest shard; counters: summed
-        memset(stats, 0, sizeof(*stats));
-        for (int i = 0; i < n_use; ++i) {
-            for (int k = 0; k < SCDE_B200_T_COUNT; ++k) {
-                if (sst[i].ms[k] > stats->ms[k]) stats->ms[k] = sst[i].ms[k];
-                stats->launches[k] += sst[i].launches[k];
-            }
-            stats->table_rows += sst[i].table_rows;
-            stats->contract_cells += sst[i].contract_cells;
-        }
-    }
-    return SCDE_B200_OK;
 }
 
 extern "C" {
@@ -2272,15 +2379,26 @@ int scde_b200_expression_difference(scde_b200_ctx *ctx, const scde_b200_diff_arg
         set_error("expression_difference: a cZ output needs the matching Z output");
         return SCDE_B200_EINVAL;
     }
-    const int r = !ctx->children.empty() ? expression_difference_multi(ctx, args, out, stats)
-                                         : expression_difference_single(ctx, args, out, stats, nullptr);
-    if (r != SCDE_B200_OK) return r;
-    // Benjamini-Hochberg over the genes of this call, once, on the host (all shards of a multi-device call have landed)
-    const int n = (args->gene_begin == 0 && args->gene_end == 0) ? args->n_genes : args->gene_end - args->gene_begin;
-    const bool has_batch = args->batch != nullptr && args->n_batch_levels > 1;
-    if (out->cz) scde::bh_cz(out->z, n, out->cz);
-    if (has_batch && out->batch_cz) scde::bh_cz(out->batch_z, n, out->batch_cz);
-    if (has_batch && out->adjusted_cz) scde::bh_cz(out->adjusted_z, n, out->adjusted_cz);
+    int g0 = 0, g1 = 0;
+    TRY(gene_range(args, &g0, &g1));
+    // Several devices: contiguous gene ranges, one per device (the split the reference's chunk() makes for n.cores,
+    // R/functions.R:606), every shard with the same Seed and therefore the same draws -- the n.cores = 1 semantics, so the
+    // result does not depend on the number of devices.  No inter-GPU traffic: every shard's results go to its rows of the
+    // caller's buffers by device-to-host copies.
+    const std::vector<scde_b200_ctx *> devs = context_devices(ctx);
+    const int n = g1 - g0;
+    const int n_use = (int)devs.size() < n ? (int)devs.size() : n;
+    std::vector<scde_b200_stats> sst(n_use);
+    TRY(on_shards(n_use, devs, [&](int i) -> int {
+        int b = 0, e = 0;
+        shard_range(n, n_use, i, &b, &e);
+        scde_b200_diff_args a = *args;
+        a.gene_begin = g0 + b;
+        a.gene_end = g0 + e;
+        return expression_difference_single(devs[i], &a, out, stats ? &sst[i] : nullptr, OutPlace{n, b});
+    }, &sst, stats));
+    // Benjamini-Hochberg over the genes of this call, once, on the host (all shards have landed)
+    bh_outputs(out, args->batch != nullptr && args->n_batch_levels > 1, n);
     return SCDE_B200_OK;
 }
 
@@ -2311,9 +2429,8 @@ struct ContrastPlan {
     std::vector<int> pair_slot, pair_bslot;  // 2 per contrast
     std::vector<int32_t> zi, zi_adj;  // n_zero entries each (1 or N)
     int n_zero = 1;
-    const double *batch_models = nullptr;
-    int b_local_theta = 0, b_sqlogit = 0;
-    bool b_fast_theta = false;
+    const double *batch_models = nullptr;  // when the call's batch.models differ from the dataset's models
+    int batch_local_theta = 0, batch_sqlogit = 0;
 };
 
 }  // namespace
@@ -2322,10 +2439,9 @@ struct ContrastPlan {
 struct DatasetShard {
     scde_b200_ctx *ctx = nullptr;
     int g0 = 0, G = 0, C = 0, K = 0;
-    int local_theta = 0, sqlogit = 0;
-    bool fast_theta = false;
     DiffWorkspace *ws = nullptr;
-    DBuf<double> models, mag, prior_y, bmodels;
+    ModelSet models, bmodels;
+    DBuf<double> mag, prior_y;
     // what the table rows hold: built from `models` (0) or from a call's batch.models (1), for the tcgen05 kernel
     // (fixed-point planes) or the FP64 kernels (FP64 rows)
     int rows_from = 0;
@@ -2357,21 +2473,14 @@ namespace {
 
 // rebuild the table rows from the models (from_batch = 0) or from the call's batch.models (1) for the kernel the context
 // selects now, unless they already are
-int ensure_rows(DatasetShard &sh, const ContrastPlan &p, int from_batch, StageTimer *tm) {
+int ensure_rows(DatasetShard &sh, int from_batch, StageTimer *tm) {
     scde_b200_ctx *ctx = sh.ctx;
     LpTable &t = sh.ws->table;
     const bool i8 = want_i8(ctx);
     if (sh.rows_from == from_batch && sh.rows_i8 == i8 && !from_batch) return SCDE_B200_OK;
     t.want_q = i8;
     sh.rows_from = -1;  // unknown until the rebuild has been queued
-    if (from_batch) {
-        t.fast_theta = p.b_fast_theta;
-        const int r = fill_table(ctx, t, sh.bmodels.p, sh.C, sh.mag.p, p.b_local_theta, p.b_sqlogit, tm);
-        t.fast_theta = sh.fast_theta;
-        TRY(r);
-    } else {
-        TRY(fill_table(ctx, t, sh.models.p, sh.C, sh.mag.p, sh.local_theta, sh.sqlogit, tm));
-    }
+    TRY(fill_rows(ctx, t, from_batch ? sh.bmodels : sh.models, sh.mag.p, tm));
     sh.rows_from = from_batch;
     sh.rows_i8 = i8;
     return SCDE_B200_OK;
@@ -2380,50 +2489,31 @@ int ensure_rows(DatasetShard &sh, const ContrastPlan &p, int from_batch, StageTi
 int shard_create(scde_b200_ctx *ctx, const scde_b200_dataset_args *a, int g0, int g1, DatasetShard **out) {
     CHECK_CTX(ctx);
     *out = nullptr;
-    if (ctx->ws_busy) {
-        set_error("another expression_difference job is alive on this context (free it first)");
-        return SCDE_B200_EINVAL;
-    }
-    if (!ctx->ws) ctx->ws = new DiffWorkspace();
+    TRY(acquire_workspace(ctx));
     DatasetShard *sh = new DatasetShard();
     sh->ctx = ctx;  // from here on, deleting the shard releases the workspace
-    ctx->ws_busy = true;
     sh->ws = ctx->ws;
     const int G = g1 - g0, C = a->n_cells, K = a->n_grid;
     sh->g0 = g0;
     sh->G = G;
     sh->C = C;
     sh->K = K;
-    sh->local_theta = a->local_theta;
-    sh->sqlogit = a->square_logit_conc;
-    sh->fast_theta = !a->local_theta && theta_all_regular(a->models, C, C);
     cudaStream_t st = ctx->stream;
     auto body = [&]() -> int {
         SCDE_CUDA(sh->ws->counts.ensure((size_t)G * C));
         SCDE_CUDA(cudaMemcpy2DAsync(sh->ws->counts.p, sizeof(int32_t) * G, a->counts + g0, sizeof(int32_t) * (size_t)a->n_genes,
                                     sizeof(int32_t) * G, C, cudaMemcpyHostToDevice, st));
-        TRY(upload(sh->models, a->models, (size_t)C * 12, st));
+        TRY(upload_models(sh->models, a->models, C, a->local_theta, a->square_logit_conc, st));
         TRY(upload(sh->prior_y, a->prior_y, (size_t)K, st));
-        std::vector<double> mag(K);
-        for (int k = 0; k < K; ++k) {  // R/functions.R:575-577
-            double m = std::pow(10.0, a->prior_x[k]) - 1;
-            if (m < 0) m = 0;
-            mag[k] = std::log(m);
-        }
+        const std::vector<double> mag = grid_magnitudes(a->prior_x, K);
         TRY(upload(sh->mag, mag.data(), (size_t)K, st));
         LpTable &t = sh->ws->table;
-        t.K = K;
-        t.ld = table_ld(K);
-        t.sentinel = -DBL_MAX / C / 1.1;
-        t.fast_theta = sh->fast_theta;
-        t.zero_base = t.ld <= KP_TILED && ctx->opt.zero_base;
-        t.want_q = want_i8(ctx);
-        t.want_modes = false;
+        init_table(ctx, t, K, C, sh->models.fast_theta);
         StageTimer &tm = sh->timer;
         tm.reset();
         const int t_all = tm.begin(st);
         TRY(index_from_counts(ctx, t, sh->ws->counts.p, G, 0, G, C, &tm));
-        TRY(fill_table(ctx, t, sh->models.p, C, sh->mag.p, sh->local_theta, sh->sqlogit, &tm));
+        TRY(fill_rows(ctx, t, sh->models, sh->mag.p, &tm));
         tm.end(SCDE_B200_T_TOTAL, t_all, st, 0);
         sh->rows_from = 0;
         sh->rows_i8 = t.want_q;
@@ -2454,21 +2544,21 @@ int shard_contrasts(DatasetShard &sh, const ContrastPlan &p, const scde_b200_con
     SCDE_CUDA(ws->scr.total.ensure(1));
     SCDE_CUDA(cudaMemsetAsync(ws->scr.total.p, 0, sizeof(unsigned long long), st));
     const int t_all = tm.begin(st);
-    TRY(ensure_rows(sh, p, 0, &tm));
+    TRY(ensure_rows(sh, 0, &tm));
     TRY(upload(sh.cells, p.cells.data(), p.cells.size(), st));
     TRY(upload(sh.draws, p.draws.data(), p.draws.size(), st));
     if (p.has_batch) TRY(upload(sh.bdraws, p.bdraws.data(), p.bdraws.size(), st));
     {
-        std::vector<int32_t> zi(p.n_zero == 1 ? 1 : G);
-        for (size_t i = 0; i < zi.size(); ++i) zi[i] = p.zi[p.n_zero == 1 ? 0 : sh.g0 + i];
+        const std::vector<int32_t> zi = zero_slice(p.zi.data(), p.n_zero, sh.g0, G);
         TRY(upload(sh.zi, zi.data(), zi.size(), st));
         if (p.has_batch) {
-            for (size_t i = 0; i < zi.size(); ++i) zi[i] = p.zi_adj[p.n_zero == 1 ? 0 : sh.g0 + i];
-            TRY(upload(sh.zi_adj, zi.data(), zi.size(), st));
+            const std::vector<int32_t> za = zero_slice(p.zi_adj.data(), p.n_zero, sh.g0, G);
+            TRY(upload(sh.zi_adj, za.data(), za.size(), st));
         }
         SCDE_CUDA(cudaStreamSynchronize(st));  // the host vectors above go out of scope
     }
-    if (p.has_batch && p.batch_models) TRY(upload(sh.bmodels, p.batch_models, (size_t)sh.C * 12, st));
+    if (p.has_batch && p.batch_models)
+        TRY(upload_models(sh.bmodels, p.batch_models, sh.C, p.batch_local_theta, p.batch_sqlogit, st));
     const size_t slot_sz = (size_t)G * ld;
     SCDE_CUDA(sh.bank.ensure((size_t)n_slots * slot_sz));
     if (p.has_batch) SCDE_CUDA(sh.bbank.ensure((size_t)n_bslots * slot_sz));
@@ -2494,7 +2584,7 @@ int shard_contrasts(DatasetShard &sh, const ContrastPlan &p, const scde_b200_con
         SCDE_CUDA(keep_flag(s));
     }
     if (p.has_batch) {
-        if (p.batch_models) TRY(ensure_rows(sh, p, 1, &tm));
+        if (p.batch_models) TRY(ensure_rows(sh, 1, &tm));
         // distinct compositions in pairs: one launch of the tcgen05 kernel for two joints over the same cells and rows
         for (int b = 0; b < n_bslots; b += 2) {
             TRY(reset_flags(ctx));
@@ -2522,28 +2612,21 @@ int shard_contrasts(DatasetShard &sh, const ContrastPlan &p, const scde_b200_con
         any = any || (f & (1 | 4));
     }
     if (any) {  // only the flagged joints are repeated, on the FP64 kernel (FP64 table rows)
-        const int keep = ctx->opt.contract_kernel;
-        ctx->opt.contract_kernel = 2;
-        auto rerun = [&]() -> int {
-            bool rows = false;
-            for (int s = 0; s < n_slots; ++s)
-                if (flags[s] & (1 | 4)) {
-                    if (!rows) TRY(ensure_rows(sh, p, 0, &tm));
-                    rows = true;
-                    TRY(group_joint(s, false));
-                }
-            rows = false;
-            for (int b = 0; b < n_bslots; ++b)
-                if (flags[n_slots + b] & (1 | 4)) {
-                    if (!rows) TRY(ensure_rows(sh, p, p.batch_models ? 1 : 0, &tm));
-                    rows = true;
-                    TRY(batch_joint(b, false, nullptr, nullptr));
-                }
-            return SCDE_B200_OK;
-        };
-        const int r = rerun();
-        ctx->opt.contract_kernel = keep;
-        TRY(r);
+        const Fp64Rerun f64(ctx);
+        bool rows = false;
+        for (int s = 0; s < n_slots; ++s)
+            if (flags[s] & (1 | 4)) {
+                if (!rows) TRY(ensure_rows(sh, 0, &tm));
+                rows = true;
+                TRY(group_joint(s, false));
+            }
+        rows = false;
+        for (int b = 0; b < n_bslots; ++b)
+            if (flags[n_slots + b] & (1 | 4)) {
+                if (!rows) TRY(ensure_rows(sh, p.batch_models ? 1 : 0, &tm));
+                rows = true;
+                TRY(batch_joint(b, false, nullptr, nullptr));
+            }
     }
     // ratio and summary: every contrast in one launch per pass; the 2K-1 posteriors that feed the adjusted pass (or that
     // the caller wants) exist only for a block of contrasts at a time, sized to the free device memory
@@ -2594,39 +2677,15 @@ int shard_contrasts(DatasetShard &sh, const ContrastPlan &p, const scde_b200_con
     }
     TRY(upload(sh.rtab, tab.data(), tab.size(), st));
     const int64_t N = p.N;
+    RatioPasses r = ratio_passes(G, K, ld, sh.prior_y.p, sh.zi.p, sh.zi_adj.p, p.n_zero);
     for (int c0 = 0; c0 < nc; c0 += nb) {
         const int n = nc - c0 < nb ? nc - c0 : nb;
         const int e0 = tm.begin(st);
-        RatioArgs r{};
-        r.ld = ld;
-        r.n_genes = G;
-        r.n = K;
-        r.prior = sh.prior_y.p;
-        r.zero_index = sh.zi.p;
-        r.n_zero = p.n_zero == 1 ? 1 : G;
-        r.ld_post = ldo;
-        r.contrasts = sh.rtab.p + c0;
-        r.n_contrasts = n;
-        SCDE_CUDA(launch_ratio_summary(r, st));
-        if (p.has_batch) {
-            // batch.effect with the default expectation = 0 (R/functions.R:362): H0 index = centre of the grid
-            RatioArgs b = r;
-            b.zero_index = nullptr;
-            b.n_zero = 1;
-            b.contrasts = sh.rtab.p + nc + c0;
-            SCDE_CUDA(launch_ratio_summary(b, st));
-            // batch adjustment: the two 2K-1 posteriors slid without prior weighting (R/functions.R:391)
-            RatioArgs a{};
-            a.ld = ldo;
-            a.n_genes = G;
-            a.n = nout;
-            a.zero_index = sh.zi_adj.p;
-            a.n_zero = p.n_zero == 1 ? 1 : G;
-            a.ld_post = lda;
-            a.contrasts = sh.rtab.p + 2 * nc + c0;
-            a.n_contrasts = n;
-            SCDE_CUDA(launch_ratio_summary(a, st));
-        }
+        r.main.contrasts = sh.rtab.p + c0;
+        r.batch.contrasts = sh.rtab.p + nc + c0;
+        r.adjusted.contrasts = sh.rtab.p + 2 * nc + c0;
+        r.main.n_contrasts = r.batch.n_contrasts = r.adjusted.n_contrasts = n;
+        TRY(launch_ratio_passes(r, p.has_batch, st));
         tm.end(SCDE_B200_T_RATIO, e0, st, n_pass);
         for (int c = c0; c < c0 + n && p.want_post; ++c) {
             const size_t k = (size_t)(c - c0);
@@ -2639,106 +2698,20 @@ int shard_contrasts(DatasetShard &sh, const ContrastPlan &p, const scde_b200_con
         }
     }
     tm.end(SCDE_B200_T_TOTAL, t_all, st, 0);
-    auto get_idx = [&](int32_t *dst, const int32_t *src) {  // [3][G] -> rows g0.. of the N x 3 block
-        return cudaMemcpy2DAsync(dst + sh.g0, sizeof(int32_t) * (size_t)N, src, sizeof(int32_t) * (size_t)G,
-                                 sizeof(int32_t) * (size_t)G, 3, cudaMemcpyDeviceToHost, st);
-    };
-    auto get_z = [&](double *dst, const double *src) {
-        return cudaMemcpyAsync(dst + sh.g0, src, sizeof(double) * (size_t)G, cudaMemcpyDeviceToHost, st);
-    };
+    const OutPlace pl{N, sh.g0};
     for (int c = 0; c < nc; ++c) {
-        const size_t i3 = (size_t)c * 3 * G, i1 = (size_t)c * G, o3 = (size_t)c * 3 * N, o1 = (size_t)c * N;
-        if (o->idx) SCDE_CUDA(get_idx(o->idx + o3, sh.idx.p + i3));
-        if (o->z) SCDE_CUDA(get_z(o->z + o1, sh.z.p + i1));
+        const size_t i3 = (size_t)c * 3 * G, i1 = (size_t)c * G;
+        TRY(download_summary(st, G, sh.idx.p + i3, sh.z.p + i1, o->idx, o->z, pl, c));
         if (!p.has_batch) continue;
-        if (o->batch_idx) SCDE_CUDA(get_idx(o->batch_idx + o3, sh.bidx.p + i3));
-        if (o->batch_z) SCDE_CUDA(get_z(o->batch_z + o1, sh.bz.p + i1));
-        if (o->adjusted_idx) SCDE_CUDA(get_idx(o->adjusted_idx + o3, sh.aidx.p + i3));
-        if (o->adjusted_z) SCDE_CUDA(get_z(o->adjusted_z + o1, sh.az.p + i1));
+        TRY(download_summary(st, G, sh.bidx.p + i3, sh.bz.p + i1, o->batch_idx, o->batch_z, pl, c));
+        TRY(download_summary(st, G, sh.aidx.p + i3, sh.az.p + i1, o->adjusted_idx, o->adjusted_z, pl, c));
     }
     if (o->joint_posteriors)
         for (int s = 0; s < n_slots; ++s)
             TRY(download_matrix(ctx, ws, G, sh.bank.p + s * slot_sz, ld, K,
-                                o->joint_posteriors + (size_t)p.slot_group[s] * N * K, OutPlace{N, sh.g0}));
+                                o->joint_posteriors + (size_t)p.slot_group[s] * N * K, pl));
     SCDE_CUDA(cudaStreamSynchronize(st));
-    if (stats) {
-        tm.collect(stats);
-        stats->table_rows = t.n_rows;
-        unsigned long long tot = 0;
-        SCDE_CUDA(cudaMemcpy(&tot, ws->scr.total.p, sizeof(tot), cudaMemcpyDeviceToHost));
-        stats->contract_cells = (int64_t)tot;
-    }
-    return SCDE_B200_OK;
-}
-
-// shard i of n over genes [0, N): the split of expression_difference_multi
-void shard_range(int N, int n, int i, int *b, int *e) {
-    const int base = N / n, rem = N % n;
-    *b = i * base + (i < rem ? i : rem);
-    *e = *b + base + (i < rem ? 1 : 0);
-}
-
-// Runs f(i) for i < n on one host thread each (directly when n == 1); exceptions become return codes, the first failing
-// shard's error text becomes this thread's.
-template <class F>
-int on_shards(int n, const std::vector<scde_b200_ctx *> &devs, F f, std::vector<scde_b200_stats> *sst, scde_b200_stats *stats) {
-    std::vector<int> rc(n, SCDE_B200_OK);
-    std::vector<std::string> msg(n);
-    auto body = [&](int i) {
-        try {
-            rc[i] = f(i);
-            if (rc[i] != SCDE_B200_OK) msg[i] = g_err;  // the error text is thread-local
-        } catch (const std::bad_alloc &) {
-            rc[i] = SCDE_B200_ENOMEM;
-            msg[i] = "host allocation failed";
-        } catch (const std::exception &ex) {
-            rc[i] = SCDE_B200_EINVAL;
-            msg[i] = ex.what();
-        } catch (...) {
-            rc[i] = SCDE_B200_EINVAL;
-            msg[i] = "unknown exception";
-        }
-    };
-    if (n == 1) {
-        body(0);
-    } else {
-        std::vector<std::thread> th;
-        try {
-            for (int i = 0; i < n; ++i) th.emplace_back(body, i);
-        } catch (...) {
-            for (auto &t : th) t.join();
-            set_error("could not start a host thread per device");
-            return SCDE_B200_ENOMEM;
-        }
-        for (auto &t : th) t.join();
-    }
-    cudaSetDevice(devs[0]->device);
-    for (int i = 0; i < n; ++i)
-        if (rc[i] != SCDE_B200_OK) {
-            if (n == 1)
-                g_err = msg[i];
-            else
-                set_error("device %d (shard %d of %d): %s", devs[i]->device, i, n, msg[i].c_str());
-            return rc[i];
-        }
-    if (stats && sst) {  // stage times: the slowest shard; counters: summed
-        memset(stats, 0, sizeof(*stats));
-        for (int i = 0; i < n; ++i) {
-            for (int k = 0; k < SCDE_B200_T_COUNT; ++k) {
-                if ((*sst)[i].ms[k] > stats->ms[k]) stats->ms[k] = (*sst)[i].ms[k];
-                stats->launches[k] += (*sst)[i].launches[k];
-            }
-            stats->table_rows += (*sst)[i].table_rows;
-            stats->contract_cells += (*sst)[i].contract_cells;
-        }
-    }
-    return SCDE_B200_OK;
-}
-
-std::vector<scde_b200_ctx *> context_devices(scde_b200_ctx *ctx) {
-    std::vector<scde_b200_ctx *> devs{ctx};
-    for (auto *c : ctx->children) devs.push_back(c);
-    return devs;
+    return collect_stats(tm, ws, stats);
 }
 
 // validation of a contrasts call and everything about it that does not depend on the device
@@ -2770,12 +2743,11 @@ int plan_contrasts(const scde_b200_dataset *ds, const scde_b200_contrast_args *a
         return bad("contrasts: zero_index (and zero_index_adjusted with batch) are required");
     TRY(validate_index(a->zero_index, (size_t)a->n_zero, 1, 2 * K, "zero_index"));
     p.zi.assign(a->zero_index, a->zero_index + a->n_zero);
+    BatchPools bp;  // the draw pools of the batch joints below
     if (p.has_batch) {
         TRY(validate_index(a->zero_index_adjusted, (size_t)a->n_zero, 1, 4 * K - 2, "zero_index_adjusted"));
         p.zi_adj.assign(a->zero_index_adjusted, a->zero_index_adjusted + a->n_zero);
-        for (int c = 0; c < C; ++c)
-            if (a->batch[c] >= a->n_batch_levels)
-                return bad("batch[%d] = %d outside [0, %d) (negative = NA)", c, a->batch[c], a->n_batch_levels);
+        TRY(batch_pools(a->batch, C, a->n_batch_levels, bp));
     }
     p.C = C;
     p.K = K;
@@ -2824,36 +2796,21 @@ int plan_contrasts(const scde_b200_dataset *ds, const scde_b200_contrast_args *a
         p.draw_off.push_back(it->second);
     }
     if (!p.has_batch) return SCDE_B200_OK;
-    // batch joints: one per distinct composition table(batch[group]) (R/functions.R:355-357), pools over all cells with a
-    // non-NA batch (tapply(seq_len(n) - 1, batch, I), :570)
+    // batch joints: one per distinct composition table(batch[group]) (R/functions.R:355-357)
     const int L = a->n_batch_levels;
-    std::vector<int32_t> off(L + 1, 0), pool;
-    for (int c = 0; c < C; ++c)
-        if (a->batch[c] >= 0) off[a->batch[c] + 1]++;
-    for (int l = 0; l < L; ++l) off[l + 1] += off[l];
-    pool.resize(off[L] > 0 ? off[L] : 1);
-    {
-        std::vector<int32_t> pos(off.begin(), off.end() - 1);
-        for (int c = 0; c < C; ++c)
-            if (a->batch[c] >= 0) pool[pos[a->batch[c]]++] = c;
-    }
     std::map<std::vector<int32_t>, int> bslot_of;
     std::vector<int> bslot_of_slot(p.slot_group.size());
     for (size_t s = 0; s < p.slot_group.size(); ++s) {
-        std::vector<int32_t> comp(L, 0);
-        int D = 0;
-        for (int64_t i = p.cell_off[s]; i < p.cell_off[s + 1]; ++i)
-            if (a->batch[p.cells[i]] >= 0) {
-                comp[a->batch[p.cells[i]]]++;
-                ++D;
-            }
+        std::vector<int32_t> comp;
+        const int D = batch_composition(a->batch, L, p.cells.data() + p.cell_off[s], (size_t)(p.cell_off[s + 1] - p.cell_off[s]),
+                                        comp);
         auto it = bslot_of.find(comp);
         if (it == bslot_of.end()) {
             it = bslot_of.emplace(comp, (int)p.bslot_D.size()).first;
             p.bslot_D.push_back(D);
             p.bdraw_off.push_back((int64_t)p.bdraws.size());
             p.bdraws.resize(p.bdraws.size() + (size_t)a->n_boot * D);
-            TRY(scde_b200_batch_boot_indices(a->seed, L, off.data(), pool.data(), comp.data(), a->n_boot,
+            TRY(scde_b200_batch_boot_indices(a->seed, L, bp.off.data(), bp.pool.data(), comp.data(), a->n_boot,
                                              p.bdraws.data() + p.bdraw_off.back()));
         }
         bslot_of_slot[s] = it->second;
@@ -2862,9 +2819,8 @@ int plan_contrasts(const scde_b200_dataset *ds, const scde_b200_contrast_args *a
     for (size_t i = 0; i < p.pair_slot.size(); ++i) p.pair_bslot[i] = bslot_of_slot[p.pair_slot[i]];
     if (a->batch_models) {
         p.batch_models = a->batch_models;
-        p.b_local_theta = a->batch_local_theta;
-        p.b_sqlogit = a->batch_square_logit_conc;
-        p.b_fast_theta = !a->batch_local_theta && theta_all_regular(a->batch_models, C, C);
+        p.batch_local_theta = a->batch_local_theta;
+        p.batch_sqlogit = a->batch_square_logit_conc;
     }
     return SCDE_B200_OK;
 }
@@ -2886,11 +2842,7 @@ int scde_b200_dataset_create(scde_b200_ctx *ctx, const scde_b200_dataset_args *a
         return SCDE_B200_EINVAL;
     }
     const std::vector<scde_b200_ctx *> devs = context_devices(ctx);
-    for (auto *d : devs)
-        if (d->ws_busy) {
-            set_error("another expression_difference job is alive on this context (free it first)");
-            return SCDE_B200_EINVAL;
-        }
+    for (auto *d : devs) TRY(workspace_busy(d));
     const int n = (int)devs.size() < a->n_genes ? (int)devs.size() : a->n_genes;
     scde_b200_dataset *ds = new scde_b200_dataset();
     ds->owner = ctx;
@@ -2943,13 +2895,7 @@ int scde_b200_dataset_contrasts(scde_b200_ctx *ctx, scde_b200_dataset *ds, const
     std::vector<scde_b200_stats> sst(n);
     TRY(on_shards(n, devs, [&](int i) -> int { return shard_contrasts(*ds->shards[i], p, o, &sst[i]); }, &sst, stats));
     // Benjamini-Hochberg per contrast over all genes, on the host, once every shard has landed
-    const int N = ds->n_genes;
-    for (int c = 0; c < a->n_contrasts; ++c) {
-        const size_t off = (size_t)c * N;
-        if (o->cz) scde::bh_cz(o->z + off, N, o->cz + off);
-        if (p.has_batch && o->batch_cz) scde::bh_cz(o->batch_z + off, N, o->batch_cz + off);
-        if (p.has_batch && o->adjusted_cz) scde::bh_cz(o->adjusted_z + off, N, o->adjusted_cz + off);
-    }
+    for (int c = 0; c < a->n_contrasts; ++c) bh_outputs(o, p.has_batch, ds->n_genes, c);
     return SCDE_B200_OK;
 }
 
