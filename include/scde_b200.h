@@ -376,6 +376,20 @@ SCDE_B200_API int scde_b200_expression_prior(scde_b200_ctx *ctx, const double *m
 SCDE_B200_API int scde_b200_cell_table(scde_b200_ctx *ctx, const double *model_row12, const int32_t *unique_counts,
                          int32_t n_counts, const double *magnitudes, int32_t n_grid, int32_t local_theta,
                          int32_t square_logit_conc, int32_t n_cells_for_clamp, double *out, int32_t *modes);
+/* The table of n_cells cells as the differential-expression call builds it for the tcgen05 contraction (zero-base form,
+ * fixed-point planes, the context's options): models[n_cells x 12] column-major; each cell's distinct counts ascending in
+ * ucl_flat[ucl_offsets[c] .. ucl_offsets[c + 1]), with or without a 0.  Outputs:
+ *   q_out[n_rows][512 * ceil(n_grid / 102)]  the planes of every row, in the layout of scde_b200_probe_contract_i8: a
+ *                                            zero-count row holds lp(0), every other row lp(x) - lp(0) of its cell (lp(x)
+ *                                            when the cell is not based), up to a constant per row; "log 0" digits are 0;
+ *   row_range_out[n_rows]                    first | last << 16 grid point that is not "log 0", or 0xFFFFFFFF;
+ *   zero_row_out[n_cells], based_out[n_cells] the cell's zero-count row (-1: none) and whether that row is free of "log 0";
+ *   zero_rows_out[n_cells][n_grid]           the zero-count row in FP64 (NaN for a cell without one).
+ * n_rows = ucl_offsets[n_cells] >= 1; n_grid <= 408 (SCDE_B200_EINVAL otherwise: no fixed-point table exists). */
+SCDE_B200_API int scde_b200_probe_table(scde_b200_ctx *ctx, const double *models, int32_t n_cells, const int32_t *ucl_flat,
+                         const int32_t *ucl_offsets, const double *magnitudes, int32_t n_grid, int32_t local_theta,
+                         int32_t square_logit_conc, int32_t n_cells_for_clamp, int8_t *q_out, uint32_t *row_range_out,
+                         int32_t *zero_row_out, int32_t *based_out, double *zero_rows_out);
 /* Measured FP64 FMA throughput of this device (TFLOP/s) from a register-resident DFMA loop; the roofline
  * denominator for the contraction kernel (MEASURED_PEAKS.json has no FP64 entry). */
 SCDE_B200_API int scde_b200_measure_fp64_peak(scde_b200_ctx *ctx, double *tflops);

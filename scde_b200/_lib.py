@@ -109,7 +109,7 @@ EXPORTED = [
     "scde_b200_jpmat_log_batch_boot", "scde_b200_mat_slide_mult", "scde_b200_ratio_posterior_summary",
     "scde_b200_bh_cz", "scde_b200_expression_difference", "scde_b200_diff_upload", "scde_b200_diff_run",
     "scde_b200_diff_download", "scde_b200_diff_free", "scde_b200_expression_magnitude", "scde_b200_cell_table",
-    "scde_b200_measure_fp64_peak", "scde_b200_set_contract_kernel", "scde_b200_probe_contract_i8",
+    "scde_b200_measure_fp64_peak", "scde_b200_set_contract_kernel", "scde_b200_probe_contract_i8", "scde_b200_probe_table",
     "scde_b200_failure_probability", "scde_b200_expression_prior", "scde_b200_dataset_create",
     "scde_b200_dataset_contrasts", "scde_b200_dataset_free",
 ]
@@ -151,6 +151,8 @@ def lib():
         L.scde_b200_dataset_free.restype = None
         L.scde_b200_create_multi.argtypes = [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_void_p)]
         L.scde_b200_n_devices.argtypes = [C.c_void_p]
+        L.scde_b200_probe_table.argtypes = [C.c_void_p, f64p, C.c_int32, i32p, i32p, f64p, C.c_int32, C.c_int32, C.c_int32,
+                                            C.c_int32, C.c_void_p, C.c_void_p, i32p, i32p, f64p]
         L.scde_b200_get_options.argtypes = [C.c_void_p, C.POINTER(Options)]
         L.scde_b200_set_options.argtypes = [C.c_void_p, C.POINTER(Options)]
         _lib = L

@@ -1094,6 +1094,78 @@ int scde_b200_cell_table(scde_b200_ctx *ctx, const double *model_row12, const in
     return SCDE_B200_OK;
 }
 
+// The table the fused path builds (fill_table in the zero-base form with fixed-point planes), copied out as it lies on the
+// device: the row kernels and the quantize pass the context's options select, nothing else.
+int scde_b200_probe_table(scde_b200_ctx *ctx, const double *models, int32_t n_cells, const int32_t *ucl_flat,
+                          const int32_t *ucl_offsets, const double *magnitudes, int32_t n_grid, int32_t local_theta,
+                          int32_t square_logit_conc, int32_t n_cells_for_clamp, int8_t *q_out, uint32_t *row_range_out,
+                          int32_t *zero_row_out, int32_t *based_out, double *zero_rows_out) {
+    CHECK_CTX(ctx);
+    if (!models || !ucl_flat || !ucl_offsets || !magnitudes || !q_out || !row_range_out || !zero_row_out || !based_out ||
+        !zero_rows_out || n_cells < 1 || n_grid < 1 || n_cells_for_clamp < 1 || ucl_offsets[0] != 0) {
+        set_error("probe_table: bad arguments");
+        return SCDE_B200_EINVAL;
+    }
+    if (n_grid > Q_MAX_K) {
+        set_error("probe_table: no fixed-point table for %d grid points (at most %d)", n_grid, Q_MAX_K);
+        return SCDE_B200_EINVAL;
+    }
+    for (int c = 0; c < n_cells; ++c) {
+        if (ucl_offsets[c + 1] < ucl_offsets[c]) {
+            set_error("probe_table: ucl_offsets not monotone at cell %d", c);
+            return SCDE_B200_EINVAL;
+        }
+        for (int r = ucl_offsets[c]; r < ucl_offsets[c + 1]; ++r)
+            if (ucl_flat[r] < 0 || (r > ucl_offsets[c] && ucl_flat[r] <= ucl_flat[r - 1])) {
+                set_error("probe_table: the counts of cell %d are not distinct, ascending and >= 0", c);
+                return SCDE_B200_EINVAL;
+            }
+    }
+    if (ucl_offsets[n_cells] < 1) {
+        set_error("probe_table: no table rows");
+        return SCDE_B200_EINVAL;
+    }
+    cudaStream_t st = ctx->stream;
+    LpTable t;
+    t.n_cells = n_cells;
+    t.K = n_grid;
+    t.ld = table_ld(n_grid);
+    t.n_rows = ucl_offsets[n_cells];
+    t.sentinel = -DBL_MAX / n_cells_for_clamp / 1.1;
+    t.fast_theta = !local_theta && theta_all_regular(models, n_cells, n_cells);
+    t.zero_base = true;
+    t.want_q = true;
+    t.want_modes = false;
+    DBuf<double> d_models, d_mag;
+    TRY(upload(d_models, models, (size_t)n_cells * 12, st));
+    TRY(upload(d_mag, magnitudes, (size_t)n_grid, st));
+    TRY(upload(t.row_off, ucl_offsets, (size_t)n_cells + 1, st));
+    TRY(upload(t.row_x, ucl_flat, (size_t)t.n_rows, st));
+    TRY(fill_table(ctx, t, d_models.p, n_cells, d_mag.p, local_theta, square_logit_conc, nullptr));
+    if (!t.has_q) {
+        set_error("probe_table: the table was built without fixed-point planes");
+        return SCDE_B200_EINVAL;
+    }
+    SCDE_CUDA(cudaMemcpyAsync(q_out, t.q.p, (size_t)t.n_rows * q_row_bytes(n_grid), cudaMemcpyDeviceToHost, st));
+    SCDE_CUDA(cudaMemcpyAsync(row_range_out, t.qrange.p, sizeof(uint32_t) * t.n_rows, cudaMemcpyDeviceToHost, st));
+    SCDE_CUDA(cudaMemcpyAsync(zero_row_out, t.zero_row.p, sizeof(int32_t) * n_cells, cudaMemcpyDeviceToHost, st));
+    SCDE_CUDA(cudaMemcpyAsync(based_out, t.based.p, sizeof(int32_t) * n_cells, cudaMemcpyDeviceToHost, st));
+    SCDE_CUDA(cudaStreamSynchronize(st));
+    // compact form: the FP64 table holds the zero-count row of cell c in slot c; otherwise in row zero_row[c]
+    for (int c = 0; c < n_cells; ++c) {
+        double *dst = zero_rows_out + (size_t)c * n_grid;
+        const int zr = zero_row_out[c];
+        if (zr < 0) {
+            for (int k = 0; k < n_grid; ++k) dst[k] = std::nan("");
+            continue;
+        }
+        const size_t slot = t.zero_compact ? (size_t)c : (size_t)zr;
+        SCDE_CUDA(cudaMemcpyAsync(dst, t.table.p + slot * t.ld, sizeof(double) * n_grid, cudaMemcpyDeviceToHost, st));
+    }
+    SCDE_CUDA(cudaStreamSynchronize(st));
+    return SCDE_B200_OK;
+}
+
 // --------------------------------------------------------------------------------------------
 static int log_boot_impl(scde_b200_ctx *ctx, const double *models, int32_t n_cells, const int32_t *ucl_flat,
                            const int32_t *ucl_offsets, const int32_t *uci, int32_t n_genes, const double *magnitudes,
