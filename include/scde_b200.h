@@ -82,12 +82,11 @@ SCDE_B200_API void *scde_b200_stream(scde_b200_ctx *ctx);
 SCDE_B200_API int scde_b200_synchronize(scde_b200_ctx *ctx);
 
 /*
- * A context over several CUDA devices of one node: the reference's `n.cores` (R/functions.R:304,566 -- gene chunks over
- * forked workers, :606-617) becomes "n devices".  scde_b200_expression_difference on such a context shards the genes
- * into contiguous ranges, one per device, runs every shard on its own host thread with the n.cores = 1 draw semantics
- * (Seed as given, one draw set for all genes, so the result does not depend on the number of devices), and the shards'
- * results land in the caller's buffers by device-to-host copies -- no inter-GPU traffic.  devices == NULL: devices
- * 0 .. n_devices-1.  Every other entry point uses the first device of the list.
+ * A context over several CUDA devices of one node.  scde_b200_expression_difference on such a context shards the genes
+ * into contiguous ranges, one per device, runs every shard on its own host thread, and the shards' results land in the
+ * caller's buffers by device-to-host copies -- no inter-GPU traffic.  The number of devices does not change results: the
+ * draws follow the call's `seed` and `draw_chunks` (the reference's n.cores, see scde_b200_diff_args) whatever the
+ * sharding.  devices == NULL: devices 0 .. n_devices-1.  Every other entry point uses the first device of the list.
  */
 SCDE_B200_API int scde_b200_create_multi(int n_devices, const int *devices, scde_b200_ctx **out);
 /* number of devices of the context (1 for scde_b200_create) */
@@ -210,7 +209,7 @@ typedef struct {
                                 composition, as tapply / table drop NA), or NULL (no correction) */
     int32_t n_batch_levels;
     int32_t n_boot;          /* n.randomizations */
-    int32_t seed;            /* Seed handed to srand(); 1 reproduces n.cores = 1 */
+    int32_t seed;            /* Seed handed to srand(); 1 reproduces the reference (see draw_chunks for its n.cores) */
     /* optional explicit draws; NULL = generate from `seed`.  [0],[1]: group joints (local indices into the
      * group's cells, n_boot x |group|); [2],[3]: batch joints (global cell ids, n_boot x number of the group's cells with
      * a non-NA batch). */
@@ -225,7 +224,17 @@ typedef struct {
      * the order of `models`; NULL = the same models (the reference's default).  With their own column-presence flags. */
     const double *batch_models;
     int32_t batch_local_theta, batch_square_logit_conc;
+    /* The reference's n.cores (R/functions.R:606-617): scde.posteriors splits the genes into n contiguous chunks and
+     * draws every chunk's randomizations with Seed = the chunk's first gene (1-based).  With n = draw_chunks > 1 and
+     * n_genes > n, chunk i is genes [b_i, e_i) of shard_range(n_genes, n, i) (the first n_genes % n chunks one gene
+     * longer) and its draws -- of every joint, group and batch -- come from seed + b_i; otherwise one draw set from
+     * `seed` for all genes.  0 or 1: one draw set (n.cores = 1).  Chunks are over the call's n_genes, not its gene range
+     * or device shard.  < 0, or > 1 together with an explicit boot_idx: SCDE_B200_EINVAL; above
+     * SCDE_B200_MAX_DRAW_CHUNKS: SCDE_B200_ELIMIT. */
+    int32_t draw_chunks;
 } scde_b200_diff_args;
+/* the largest draw_chunks: it bounds the per-set W and Z memory and the number of host threads generating draws */
+#define SCDE_B200_MAX_DRAW_CHUNKS 256
 
 typedef struct {
     /* per processed gene; any pointer may be NULL to skip that output */
@@ -292,7 +301,7 @@ SCDE_B200_API void scde_b200_diff_free(scde_b200_ctx *ctx, scde_b200_diff_job *j
  * with the one-shot call within the oracle tolerances.
  *
  * Each group's joint posterior is computed once per call however many contrasts name it (the draws of a group depend on
- * the seed, n_boot and the group's size only), and each distinct batch composition's joint once.
+ * the seed, n_boot, draw_chunks and the group's size only), and each distinct batch composition's joint once.
  *
  * A dataset holds its context's differential-expression workspace until scde_b200_dataset_free: while it is alive,
  * scde_b200_expression_difference, scde_b200_diff_upload and a second scde_b200_dataset_create on that context fail with
@@ -324,6 +333,7 @@ typedef struct {
     int32_t n_batch_levels;
     const double *batch_models;    /* n_cells x 12 or NULL (= models), with their own column-presence flags */
     int32_t batch_local_theta, batch_square_logit_conc;
+    int32_t draw_chunks;           /* as in scde_b200_diff_args, over the dataset's n_genes */
 } scde_b200_contrast_args;
 
 /* Outputs, any pointer may be NULL.  Per-contrast blocks back to back: contrast c's block of a G x m output starts at

@@ -1,12 +1,14 @@
 # scde_b200.R -- R side of the drop-in.  With integration/scde_b200_shim.cpp in src/ (instead of jpmatLogBoot.cpp and
 # matSlideMult.cpp) scde.posteriors / scde.expression.difference / scde.test.gene.expression.difference work UNCHANGED:
 # their .Call sites resolve to the shim.  Two things to know:
-#   * call them with n.cores = 1: papply forks (R/functions.R:6054), and a CUDA context does not survive fork(); the GPU
-#     replaces the gene-chunk parallelism, and the library always draws as n.cores = 1 does (Seed = 1, one draw set);
+#   * call them with n.cores = 1: papply forks (R/functions.R:6054), and a CUDA context does not survive fork(); the
+#     shim's .Call entries draw as one call does, so results equal scde's at n.cores = 1;
 #   * for large inputs use the fused entry below: the joint posteriors (genes x 401 doubles per group) then never cross
-#     PCIe, and `n.devices` GPUs share the genes (the reference's n.cores).
+#     PCIe, `n.cores` reproduces scde's results at that n.cores (one draw set per gene chunk, computed in the same device
+#     launches, nothing forks), and `n.devices` GPUs share the genes without changing results.
 scde.expression.difference.b200 <- function(models, counts, prior, groups = NULL, batch = NULL, n.randomizations = 150,
-                                            n.devices = 1, batch.models = models, expectation = 0, devices = seq_len(n.devices) - 1L) {
+                                            n.devices = 1, batch.models = models, expectation = 0, devices = seq_len(n.devices) - 1L,
+                                            n.cores = 1) {
   if(!all(rownames(models) %in% colnames(counts))) stop("ERROR: provided count data does not cover all of the cells specified in the model matrix")
   counts <- as.matrix(counts[, match(rownames(models), colnames(counts))]); storage.mode(counts) <- "integer"
   if(is.null(groups)) { groups <- as.factor(attr(models, "groups")); names(groups) <- rownames(models) }
@@ -31,7 +33,7 @@ scde.expression.difference.b200 <- function(models, counts, prior, groups = NULL
              as.integer(groups) - 1L, if(correct.batch) as.integer(batch) - 1L else integer(0),
              if(correct.batch) length(levels(batch)) else 0L, as.integer(n.randomizations), 1L, as.integer(zidx(rv)),
              as.integer(zidx(arv)), as.integer("corr.ltheta.b" %in% colnames(models)), as.integer("conc.a2" %in% colnames(models)),
-             as.integer(devices), PACKAGE = "scde")
+             as.integer(devices), as.integer(n.cores), PACKAGE = "scde")
   if(correct.batch) names(r) <- c("idx", "z", "cz", "batch.idx", "batch.z", "batch.cz", "adjusted.idx", "adjusted.z", "adjusted.cz")
   frame <- function(idx, z, cz, grid) {                      # quick.distribution.summary, R/functions.R:5045-5052
     dq <- cbind(lb = grid[idx[, 1] + 1], mle = grid[idx[, 2] + 1], ub = grid[idx[, 3] + 1]) / log10(2)
@@ -52,7 +54,7 @@ scde.expression.difference.b200 <- function(models, counts, prior, groups = NULL
 # scde.expression.difference.b200 returns for the two-level factor (A first; cells of neither side NA).
 scde.expression.difference.contrasts.b200 <- function(models, counts, prior, groups, contrasts = NULL, batch = NULL,
                                                       n.randomizations = 150, n.devices = 1, batch.models = models,
-                                                      expectation = 0, devices = seq_len(n.devices) - 1L) {
+                                                      expectation = 0, devices = seq_len(n.devices) - 1L, n.cores = 1) {
   if(!all(rownames(models) %in% colnames(counts))) stop("ERROR: provided count data does not cover all of the cells specified in the model matrix")
   counts <- as.matrix(counts[, match(rownames(models), colnames(counts))]); storage.mode(counts) <- "integer"
   groups <- as.factor(groups); lev <- levels(groups)
@@ -100,7 +102,7 @@ scde.expression.difference.contrasts.b200 <- function(models, counts, prior, gro
              as.integer(n.randomizations), 1L, as.integer(zidx(rv)), as.integer(zidx(arv)),
              as.integer("corr.ltheta.b" %in% colnames(models)), as.integer("conc.a2" %in% colnames(models)),
              as.integer("corr.ltheta.b" %in% colnames(batch.models)), as.integer("conc.a2" %in% colnames(batch.models)),
-             as.integer(devices), PACKAGE = "scde")
+             as.integer(devices), as.integer(n.cores), PACKAGE = "scde")
   frame <- function(idx, z, cz, grid) {                      # quick.distribution.summary, R/functions.R:5045-5052
     dq <- cbind(lb = grid[idx[, 1] + 1], mle = grid[idx[, 2] + 1], ub = grid[idx[, 3] + 1]) / log10(2)
     cq <- rep(0, nrow(dq)); cq[dq[, 1] > 0] <- dq[dq[, 1] > 0, 1]; cq[dq[, 3] < 0] <- dq[dq[, 3] < 0, 3]

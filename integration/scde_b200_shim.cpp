@@ -14,8 +14,9 @@
 // tests/test_gpu_parity.py::test_r_shim_symbols_against_reference_fixtures drives the five symbols on a GPU and compares
 // them with the reference's own C++ -- the code path an R session would take, minus R.
 //
-// n.cores -> devices: SCDE_B200_DEVICES (e.g. "0,1,2,3") or the `devices` argument of scde_b200_diff selects the GPUs of
-// a multi-device context; the gene chunks of papply (R/functions.R:606-617) become gene shards inside the library.
+// Devices: SCDE_B200_DEVICES (e.g. "0,1,2,3") or the `devices` argument of scde_b200_diff selects the GPUs of a
+// multi-device context, which shards the genes without changing results.  The reference's n.cores (the gene chunks of
+// papply, R/functions.R:606-617, each with its own Seed) is the DrawChunks argument of the fused entries.
 #include <Rcpp.h>
 #include "scde_b200.h"
 
@@ -182,11 +183,13 @@ RcppExport SEXP jpmatLogBatchBoot(SEXP Matll, SEXP Comp, SEXP Nboot, SEXP Seed) 
 //   Models   numeric matrix cells x 12 (NA where a column is absent; corr.a already clamped to >= 1e-10)
 //   Group    integer vector, 0 / 1 per cell, negative = NA;   Batch: integer codes 0..L-1 (negative = NA) or length 0
 //   ZeroIndex / ZeroIndexAdjusted: 1-based H0 grid positions (length 1 or genes)
-//   Devices  integer vector of CUDA device ids (length 0: SCDE_B200_DEVICES, else device 0) -- the n.cores of the GPU path
+//   Devices  integer vector of CUDA device ids (length 0: SCDE_B200_DEVICES, else device 0); they do not change results
+//   DrawChunks  the reference's n.cores: one draw set per gene chunk, Seed = Seed + the chunk's first gene (0-based)
+//               (scde_b200_diff_args.draw_chunks; 1 = one draw set)
 // Returns list(idx, z, cz[, batch.idx, batch.z, batch.cz, adjusted.idx, adjusted.z, adjusted.cz]).
 RcppExport SEXP scde_b200_diff(SEXP Counts, SEXP Models, SEXP BatchModels, SEXP PriorX, SEXP PriorY, SEXP Group, SEXP Batch,
                                SEXP NBatchLevels, SEXP Nboot, SEXP Seed, SEXP ZeroIndex, SEXP ZeroIndexAdjusted,
-                               SEXP LocalThetaFit, SEXP SquareLogitConc, SEXP Devices) {
+                               SEXP LocalThetaFit, SEXP SquareLogitConc, SEXP Devices, SEXP DrawChunks) {
     Rcpp::IntegerMatrix counts(Counts);
     Rcpp::NumericMatrix models(Models), bmodels(BatchModels);
     Rcpp::NumericVector px(PriorX), py(PriorY);
@@ -214,6 +217,7 @@ RcppExport SEXP scde_b200_diff(SEXP Counts, SEXP Models, SEXP BatchModels, SEXP 
     a.batch_models = (has_batch && bmodels.size() == C * 12) ? bmodels.begin() : NULL;
     a.batch_local_theta = a.local_theta;
     a.batch_square_logit_conc = a.square_logit_conc;
+    a.draw_chunks = Rcpp::as<int>(DrawChunks);
     std::vector<int> idx((size_t)3 * G), bidx(has_batch ? (size_t)3 * G : 0), aidx(has_batch ? (size_t)3 * G : 0);
     Rcpp::NumericMatrix z(G, 1), bz(has_batch ? G : 0, 1), az(has_batch ? G : 0, 1);
     Rcpp::NumericMatrix cz(G, 1), bcz(has_batch ? G : 0, 1), acz(has_batch ? G : 0, 1);  // BH-corrected (R/functions.R:5051)
@@ -259,13 +263,14 @@ RcppExport SEXP scde_b200_diff(SEXP Counts, SEXP Models, SEXP BatchModels, SEXP 
 //   Pairs                      2 x n.contrasts 0-based group ids, column c = (A, B) of contrast c
 //   BatchModels                cells x 12 or a 0 x 0 matrix (= Models), with its own BatchLocalThetaFit / BatchSquareLogitConc
 //                              flags (from colnames(batch.models))
+//   DrawChunks                 as in scde_b200_diff, over the genes of Counts
 // Returns list(idx, z, cz[, batch.idx, batch.z, batch.cz, adjusted.idx, adjusted.z, adjusted.cz]): idx genes x (3 x
 // n.contrasts), contrast c in columns 3c+1 .. 3c+3 (lb, mle, ub, 0-based grid indices); z and cz genes x n.contrasts.
 RcppExport SEXP scde_b200_diff_contrasts(SEXP Counts, SEXP Models, SEXP BatchModels, SEXP PriorX, SEXP PriorY,
                                          SEXP GroupOffsets, SEXP GroupCells, SEXP Pairs, SEXP Batch, SEXP NBatchLevels,
                                          SEXP Nboot, SEXP Seed, SEXP ZeroIndex, SEXP ZeroIndexAdjusted, SEXP LocalThetaFit,
                                          SEXP SquareLogitConc, SEXP BatchLocalThetaFit, SEXP BatchSquareLogitConc,
-                                         SEXP Devices) {
+                                         SEXP Devices, SEXP DrawChunks) {
     Rcpp::IntegerMatrix counts(Counts);
     Rcpp::NumericMatrix models(Models), bmodels(BatchModels);
     Rcpp::NumericVector px(PriorX), py(PriorY);
@@ -299,6 +304,7 @@ RcppExport SEXP scde_b200_diff_contrasts(SEXP Counts, SEXP Models, SEXP BatchMod
     a.batch_models = (has_batch && bmodels.size() == C * 12) ? bmodels.begin() : NULL;
     a.batch_local_theta = Rcpp::as<int>(BatchLocalThetaFit);
     a.batch_square_logit_conc = Rcpp::as<int>(BatchSquareLogitConc);
+    a.draw_chunks = Rcpp::as<int>(DrawChunks);
     const int n_sets = has_batch ? 3 : 1;
     std::vector<int> idx((size_t)n_sets * 3 * G * nc);
     std::vector<Rcpp::NumericMatrix> z, cz;

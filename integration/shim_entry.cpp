@@ -7,12 +7,12 @@
 
 RcppExport SEXP scde_b200_diff(SEXP Counts, SEXP Models, SEXP BatchModels, SEXP PriorX, SEXP PriorY, SEXP Group, SEXP Batch,
                                SEXP NBatchLevels, SEXP Nboot, SEXP Seed, SEXP ZeroIndex, SEXP ZeroIndexAdjusted,
-                               SEXP LocalThetaFit, SEXP SquareLogitConc, SEXP Devices);
+                               SEXP LocalThetaFit, SEXP SquareLogitConc, SEXP Devices, SEXP DrawChunks);
 RcppExport SEXP scde_b200_diff_contrasts(SEXP Counts, SEXP Models, SEXP BatchModels, SEXP PriorX, SEXP PriorY,
                                          SEXP GroupOffsets, SEXP GroupCells, SEXP Pairs, SEXP Batch, SEXP NBatchLevels,
                                          SEXP Nboot, SEXP Seed, SEXP ZeroIndex, SEXP ZeroIndexAdjusted, SEXP LocalThetaFit,
                                          SEXP SquareLogitConc, SEXP BatchLocalThetaFit, SEXP BatchSquareLogitConc,
-                                         SEXP Devices);
+                                         SEXP Devices, SEXP DrawChunks);
 
 namespace {
 SEXP ivec(const int *p, size_t n) {
@@ -28,10 +28,12 @@ SEXP dvec(const double *p, size_t n) {
 }  // namespace
 
 // no batch: out_idx[G*3] (as doubles, 0-based), out_z[G], out_cz[G]; with a batch factor additionally the batch.effect and
-// batch.adjusted triples behind them (out arrays sized 3x).  Returns 0, or -1 with the message in err[256].
-extern "C" int shim_diff(const int *counts, int G, int C, const double *models12, const double *px, const double *py, int K,
-                         const int *group, const int *batch, int n_levels, int nboot, int zero_index, int zero_index_adj,
-                         const int *devices, int n_devices, double *out_idx, double *out_z, double *out_cz, char *err) {
+// batch.adjusted triples behind them (out arrays sized 3x).  draw_chunks: the DrawChunks argument (the reference's
+// n.cores).  Returns 0, or -1 with the message in err[256].
+extern "C" int shim_diff_chunked(const int *counts, int G, int C, const double *models12, const double *px, const double *py,
+                                 int K, const int *group, const int *batch, int n_levels, int nboot, int zero_index,
+                                 int zero_index_adj, const int *devices, int n_devices, int draw_chunks, double *out_idx,
+                                 double *out_z, double *out_cz, char *err) {
     int rc = 0;
     try {
         SEXP cnt = ivec(counts, (size_t)G * C);
@@ -45,7 +47,8 @@ extern "C" int shim_diff(const int *counts, int G, int C, const double *models12
         int one = 1, zero = 0;
         SEXP r = scde_b200_diff(cnt, mm, bm, dvec(px, K), dvec(py, K), ivec(group, C), ivec(batch, batch ? C : 0),
                                 ivec(&n_levels, 1), ivec(&nboot, 1), ivec(&one, 1), ivec(&zero_index, 1),
-                                ivec(&zero_index_adj, 1), ivec(&zero, 1), ivec(&zero, 1), ivec(devices, n_devices));
+                                ivec(&zero_index_adj, 1), ivec(&zero, 1), ivec(&zero, 1), ivec(devices, n_devices),
+                                ivec(&draw_chunks, 1));
         const int n_sets = (int)r->list.size() / 3;
         for (int s = 0; s < n_sets; ++s) {
             std::memcpy(out_idx + (size_t)s * 3 * G, r->list[3 * s]->dval.data(), sizeof(double) * 3 * G);
@@ -61,14 +64,23 @@ extern "C" int shim_diff(const int *counts, int G, int C, const double *models12
     return rc;
 }
 
+// one draw set (n.cores = 1)
+extern "C" int shim_diff(const int *counts, int G, int C, const double *models12, const double *px, const double *py, int K,
+                         const int *group, const int *batch, int n_levels, int nboot, int zero_index, int zero_index_adj,
+                         const int *devices, int n_devices, double *out_idx, double *out_z, double *out_cz, char *err) {
+    return shim_diff_chunked(counts, G, C, models12, px, py, K, group, batch, n_levels, nboot, zero_index, zero_index_adj,
+                             devices, n_devices, 1, out_idx, out_z, out_cz, err);
+}
+
 // scde_b200_diff_contrasts: groups as flattened 0-based cell lists, pairs[2 * n_contrasts]; batch models = models.
 // out_idx[n_sets * n_contrasts * 3 * G] (as doubles), out_z / out_cz[n_sets * n_contrasts * G], n_sets = 3 with a batch
 // factor (results, batch.effect, batch.adjusted), else 1; contrast c's block inside a set as in scde_b200_contrast_out.
-extern "C" int shim_diff_contrasts(const int *counts, int G, int C, const double *models12, const double *px, const double *py,
-                                   int K, const int *group_offsets, int n_groups, const int *group_cells, const int *pairs,
-                                   int n_contrasts, const int *batch, int n_levels, int nboot, int zero_index,
-                                   int zero_index_adj, const int *devices, int n_devices, double *out_idx, double *out_z,
-                                   double *out_cz, char *err) {
+extern "C" int shim_diff_contrasts_chunked(const int *counts, int G, int C, const double *models12, const double *px,
+                                           const double *py, int K, const int *group_offsets, int n_groups,
+                                           const int *group_cells, const int *pairs, int n_contrasts, const int *batch,
+                                           int n_levels, int nboot, int zero_index, int zero_index_adj, const int *devices,
+                                           int n_devices, int draw_chunks, double *out_idx, double *out_z, double *out_cz,
+                                           char *err) {
     int rc = 0;
     try {
         SEXP cnt = ivec(counts, (size_t)G * C);
@@ -84,7 +96,7 @@ extern "C" int shim_diff_contrasts(const int *counts, int G, int C, const double
                                           ivec(group_cells, group_offsets[n_groups]), ivec(pairs, 2 * (size_t)n_contrasts),
                                           ivec(batch, batch ? C : 0), ivec(&n_levels, 1), ivec(&nboot, 1), ivec(&one, 1),
                                           ivec(&zero_index, 1), ivec(&zero_index_adj, 1), ivec(&zero, 1), ivec(&zero, 1),
-                                          ivec(&zero, 1), ivec(&zero, 1), ivec(devices, n_devices));
+                                          ivec(&zero, 1), ivec(&zero, 1), ivec(devices, n_devices), ivec(&draw_chunks, 1));
         const int n_sets = (int)r->list.size() / 3;
         const size_t n3 = (size_t)3 * G * n_contrasts, n1 = (size_t)G * n_contrasts;
         for (int s = 0; s < n_sets; ++s) {
@@ -99,4 +111,14 @@ extern "C" int shim_diff_contrasts(const int *counts, int G, int C, const double
     }
     ShimArena::get().clear();
     return rc;
+}
+
+extern "C" int shim_diff_contrasts(const int *counts, int G, int C, const double *models12, const double *px, const double *py,
+                                   int K, const int *group_offsets, int n_groups, const int *group_cells, const int *pairs,
+                                   int n_contrasts, const int *batch, int n_levels, int nboot, int zero_index,
+                                   int zero_index_adj, const int *devices, int n_devices, double *out_idx, double *out_z,
+                                   double *out_cz, char *err) {
+    return shim_diff_contrasts_chunked(counts, G, C, models12, px, py, K, group_offsets, n_groups, group_cells, pairs,
+                                       n_contrasts, batch, n_levels, nboot, zero_index, zero_index_adj, devices, n_devices, 1,
+                                       out_idx, out_z, out_cz, err);
 }

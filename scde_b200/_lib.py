@@ -37,6 +37,7 @@ class DiffArgs(C.Structure):
         ("local_theta", C.c_int32), ("square_logit_conc", C.c_int32),
         ("gene_begin", C.c_int32), ("gene_end", C.c_int32),
         ("batch_models", f64p), ("batch_local_theta", C.c_int32), ("batch_square_logit_conc", C.c_int32),
+        ("draw_chunks", C.c_int32),
     ]
 
 
@@ -69,6 +70,7 @@ class ContrastArgs(C.Structure):
         ("zero_index", i32p), ("n_zero", C.c_int32), ("zero_index_adjusted", i32p),
         ("batch", i32p), ("n_batch_levels", C.c_int32),
         ("batch_models", f64p), ("batch_local_theta", C.c_int32), ("batch_square_logit_conc", C.c_int32),
+        ("draw_chunks", C.c_int32),
     ]
 
 

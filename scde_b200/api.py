@@ -12,8 +12,12 @@ Same function names (dots -> underscores), argument meaning and error behaviour 
 R data frames become pandas DataFrames (models: cells x coefficients; counts: genes x cells; prior: columns
 ``x`` and ``y``), factors become pandas Categoricals / Series.  All numeric work happens in libscde_b200.so
 through the C ABI (``_lib``); this module only does what the R layer does: validation, reordering, packing,
-labelling.  ``n_cores`` is accepted for signature compatibility and ignored -- the GPU path must not go through
-a fork (SURVEY.md section 7) and always has the ``n.cores = 1`` semantics (Seed = 1, one draw set for all genes).
+labelling.  Nothing forks (SURVEY.md section 7).  ``n_cores`` is the reference's n.cores, which changes results: scde
+splits the genes into n.cores chunks and draws every chunk's randomizations with its own Seed (R/functions.R:606-617).
+By default (``chunked_draws=False``) ``n_cores`` is ignored and the results are those of ``n.cores = 1`` (Seed = 1, one
+draw set for all genes).  ``chunked_draws=True`` honours it: ``scde_expression_difference`` and
+``DifferenceSession.contrasts`` compute every chunk's draw set in the same device launches (``draw_chunks`` of the C
+ABI), and ``scde_posteriors`` calls the library once per chunk, as the reference does.
 """
 from __future__ import annotations
 
@@ -34,6 +38,33 @@ MIN_SLOPE = 1e-10  # R/functions.R:579
 
 def _stop(msg: str):
     raise ValueError("ERROR: " + msg)
+
+
+def draw_chunk_ranges(G: int, n_cores: int) -> list:
+    """The gene chunks of scde.posteriors with n.cores = n_cores (R/functions.R:606-617): the 0-based ranges [b, e) of
+    split(seq_len(G), sort(rep_len(1:n, G))) when n > 1 and G > n (the first G %% n chunks one gene longer), else
+    [(0, G)].  Chunk [b, e) draws with Seed = seed + b."""
+    n = int(n_cores)
+    if not (n > 1 and G > n):
+        return [(0, G)]
+    base, rem = divmod(G, n)
+    out, b = [], 0
+    for i in range(n):
+        e = b + base + (1 if i < rem else 0)
+        out.append((b, e))
+        b = e
+    return out
+
+
+def _draw_chunks(chunked_draws: bool, n_cores: int, boot_idx) -> int:
+    """draw_chunks of the C ABI for (chunked_draws, n_cores); explicit draws cannot be chunked."""
+    if not chunked_draws:
+        return 0
+    if any(b is not None for b in (boot_idx if isinstance(boot_idx, (tuple, list)) else (boot_idx,))):
+        raise ValueError("ERROR: chunked_draws draws every gene chunk from its own seed; it cannot be combined with boot_idx")
+    if int(n_cores) < 1:
+        raise ValueError("ERROR: n_cores must be >= 1")
+    return int(n_cores)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -145,13 +176,32 @@ def scde_expression_magnitude(models: pd.DataFrame, counts) -> pd.DataFrame:
 
 def scde_posteriors(models: pd.DataFrame, counts, prior, n_randomizations: int = 100, batch=None, composition=None,
                     return_individual_posteriors: bool = False, return_individual_posterior_modes: bool = False,
-                    ensemble_posterior: bool = False, n_cores: int = 20, seed: int = 1, boot_idx=None, context=None):
+                    ensemble_posterior: bool = False, n_cores: int = 20, seed: int = 1, boot_idx=None, context=None,
+                    chunked_draws: bool = False):
     """Joint posterior of the cells in `models` (scde.posteriors, R/functions.R:566-670).
 
     Returns a genes x K DataFrame (columns = as.character(exp(marginals))) or, with the return_individual_* flags,
     a dict with ``jp`` plus ``modes`` (genes x cells) and/or ``post`` (dict cell -> genes x K DataFrame).
-    `seed` / `boot_idx` expose what the reference fixes at Seed = 1 for n.cores = 1.
+    `seed` / `boot_idx` expose what the reference fixes at Seed = 1 for n.cores = 1.  chunked_draws: one call per gene
+    chunk of ``n_cores`` (draw_chunk_ranges) with Seed = seed + the chunk's first gene, results stacked -- the
+    reference's own loop.
     """
+    if _draw_chunks(chunked_draws, n_cores, boot_idx) > 1:
+        cm, genes = _counts_for_models(models, counts)
+        chunks = draw_chunk_ranges(cm.shape[0], n_cores)
+        if len(chunks) > 1:
+            cdf = pd.DataFrame(cm, index=genes, columns=list(models.index))
+            parts = [scde_posteriors(models, cdf.iloc[b:e], prior, n_randomizations, batch, composition,
+                                     return_individual_posteriors, return_individual_posterior_modes, ensemble_posterior,
+                                     1, seed + b, None, context) for b, e in chunks]
+            if isinstance(parts[0], pd.DataFrame):
+                return pd.concat(parts)
+            out = {"jp": pd.concat([p["jp"] for p in parts])}
+            if "modes" in parts[0]:
+                out["modes"] = pd.concat([p["modes"] for p in parts])
+            if "post" in parts[0]:
+                out["post"] = {cell: pd.concat([p["post"][cell] for p in parts]) for cell in parts[0]["post"]}
+            return out
     cm, genes = _counts_for_models(models, counts)
     pools = comp = None
     if batch is not None:
@@ -342,7 +392,7 @@ def quick_distribution_summary(pmat1, pmat2, prior, expectation=0.0, skip_prior_
 # ------------------------------------------------------------------------------------------------
 def _diff_args(counts, mm, prior_x, prior_y, group_codes, n_boot, seed, batch_codes, n_batch_levels, zero_index,
                zero_index_adjusted, local_theta, sqlogit, boot_idx, gene_range, batch_mm=None, batch_local_theta=0,
-               batch_sqlogit=0):
+               batch_sqlogit=0, draw_chunks=0):
     """scde_b200_diff_args for the C ABI; returns (args, the host arrays it points into, processed genes, K, has_batch)."""
     keep_alive = []
 
@@ -375,6 +425,7 @@ def _diff_args(counts, mm, prior_x, prior_y, group_codes, n_boot, seed, batch_co
     if batch_mm is not None:
         a.batch_models = p_f64(keep(f64(batch_mm)))
         a.batch_local_theta, a.batch_square_logit_conc = int(batch_local_theta), int(batch_sqlogit)
+    a.draw_chunks = int(draw_chunks)
     G = (gene_range[1] - gene_range[0]) if tuple(gene_range) != (0, 0) else G_all
     return a, keep_alive, G, K, has_batch
 
@@ -420,12 +471,15 @@ def expression_difference_call(ctx: _lib.Context, counts: np.ndarray, mm: np.nda
                                n_boot: int, seed: int = 1, batch_codes=None, n_batch_levels: int = 0, zero_index=None,
                                zero_index_adjusted=None, local_theta: int = 0, sqlogit: int = 0, boot_idx=(None,) * 4,
                                gene_range=(0, 0), want_posteriors: bool = False, joint_posteriors: bool = False,
-                               batch_mm=None, batch_local_theta: int = 0, batch_sqlogit: int = 0):
+                               batch_mm=None, batch_local_theta: int = 0, batch_sqlogit: int = 0, n_cores: int = 1,
+                               chunked_draws: bool = False):
     """The one-shot C-ABI call (scde_b200_expression_difference): host buffers in, host buffers out.  The count matrix is
-    uploaded in cell chunks while the table rows of the chunks already on the device are being built."""
+    uploaded in cell chunks while the table rows of the chunks already on the device are being built.  chunked_draws:
+    the draws of n.cores = n_cores (see the module docstring)."""
+    dc = _draw_chunks(chunked_draws, n_cores, boot_idx)
     a, keep_alive, G, K, has_batch = _diff_args(counts, mm, prior_x, prior_y, group_codes, n_boot, seed, batch_codes,
                                                 n_batch_levels, zero_index, zero_index_adjusted, local_theta, sqlogit,
-                                                boot_idx, gene_range, batch_mm, batch_local_theta, batch_sqlogit)
+                                                boot_idx, gene_range, batch_mm, batch_local_theta, batch_sqlogit, dc)
     o, res = _diff_out(G, K, has_batch, want_posteriors, joint_posteriors, want_cz=tuple(gene_range) == (0, 0))
     st = _lib.Stats()
     check(lib().scde_b200_expression_difference(ctx.handle, C.byref(a), C.byref(o), C.byref(st)))
@@ -441,11 +495,13 @@ class DifferenceJob:
                  n_boot: int, seed: int = 1, batch_codes=None, n_batch_levels: int = 0, zero_index=None,
                  zero_index_adjusted=None, local_theta: int = 0, sqlogit: int = 0, boot_idx=(None,) * 4,
                  gene_range=(0, 0), want_posteriors: bool = False, batch_mm=None, batch_local_theta: int = 0,
-                 batch_sqlogit: int = 0):
+                 batch_sqlogit: int = 0, n_cores: int = 1, chunked_draws: bool = False):
         self.ctx = ctx
+        dc = _draw_chunks(chunked_draws, n_cores, boot_idx)
         a, keep_alive, self.G, self.K, self.has_batch = _diff_args(
             counts, mm, prior_x, prior_y, group_codes, n_boot, seed, batch_codes, n_batch_levels, zero_index,
-            zero_index_adjusted, local_theta, sqlogit, boot_idx, gene_range, batch_mm, batch_local_theta, batch_sqlogit)
+            zero_index_adjusted, local_theta, sqlogit, boot_idx, gene_range, batch_mm, batch_local_theta, batch_sqlogit,
+            dc)
         self.want_posteriors = bool(want_posteriors)
         self._job = C.c_void_p()
         check(lib().scde_b200_diff_upload(ctx.handle, C.byref(a), int(want_posteriors), C.byref(self._job)))
@@ -528,13 +584,15 @@ def _difference_result(r: dict, genes, diffv, adiffv, kcols, names, correct_batc
 def scde_expression_difference(models: pd.DataFrame, counts, prior, groups=None, batch=None,
                                n_randomizations: int = 150, n_cores: int = 10, batch_models=None,
                                return_posteriors: bool = False, expectation=0, verbose: int = 0, seed: int = 1,
-                               context=None, boot_idx=(None,) * 4):
+                               context=None, boot_idx=(None,) * 4, chunked_draws: bool = False):
     """scde.expression.difference (R/functions.R:304-408).
 
     Returns the ``lb mle ub ce Z cZ`` data frame (genes as rows), or a dict shaped like the reference's list when
     `batch` and/or `return_posteriors` are given (keys: ``results``, ``batch.adjusted``, ``batch.effect``,
     ``difference.posterior``, ``batch.adjusted.difference.posterior``, ``joint.posteriors``).
+    chunked_draws: honour n_cores as the reference's n.cores (one draw set per gene chunk; see the module docstring).
     """
+    _draw_chunks(chunked_draws, n_cores, boot_idx)  # argument errors before any library call
     cm, genes = _counts_for_models(models, counts)
     if groups is None:
         groups = models.attrs.get("groups")
@@ -578,7 +636,7 @@ def scde_expression_difference(models: pd.DataFrame, counts, prior, groups=None,
                                      n_batch_levels=len(blev) if correct_batch else 0, zero_index=zi,
                                      zero_index_adjusted=zia, local_theta=lt, sqlogit=sq, boot_idx=boot_idx,
                                      want_posteriors=return_posteriors, batch_mm=bmm, batch_local_theta=blt,
-                                     batch_sqlogit=bsq)
+                                     batch_sqlogit=bsq, n_cores=n_cores, chunked_draws=chunked_draws)
     if verbose:
         sys.stdout.write("summarizing differences\n")
     with np.errstate(over="ignore"):
@@ -728,10 +786,13 @@ class DifferenceSession:
         self.last_stats = None
 
     def contrasts(self, groups, contrasts="pairs", batch=None, batch_models=None, n_randomizations: int = 150,
-                  return_posteriors: bool = False, expectation=0, seed: int = 1) -> dict:
-        """``{"<A> vs <B>": result}``, each result what ``scde_expression_difference`` returns for that contrast."""
+                  return_posteriors: bool = False, expectation=0, seed: int = 1, n_cores: int = 1,
+                  chunked_draws: bool = False) -> dict:
+        """``{"<A> vs <B>": result}``, each result what ``scde_expression_difference`` returns for that contrast (with
+        the same n_cores and chunked_draws)."""
         if not self._ds:
             _stop("the session is closed")
+        draw_chunks = _draw_chunks(chunked_draws, n_cores, None)
         gcodes, glev = _named_factor(groups, self.models.index)
         plan = expand_contrasts(glev, contrasts)
         code_of = {lev: i for i, lev in enumerate(glev)}
@@ -772,6 +833,7 @@ class DifferenceSession:
         a.n_groups, a.group_offsets, a.group_cells = ng, p_i32(off), p_i32(cells)
         a.n_contrasts, a.pairs = nc, p_i32(pr)
         a.n_boot, a.seed = int(n_randomizations), int(seed)
+        a.draw_chunks = draw_chunks
         zi, zia = i32(zi), i32(zia)
         a.zero_index, a.n_zero, a.zero_index_adjusted = p_i32(zi), len(zi), p_i32(zia)
         bc = i32(bcodes) if correct_batch else None
@@ -826,10 +888,11 @@ class DifferenceSession:
 
 def scde_expression_difference_contrasts(models: pd.DataFrame, counts, prior, groups, contrasts="pairs", batch=None,
                                          batch_models=None, n_randomizations: int = 150, return_posteriors: bool = False,
-                                         expectation=0, seed: int = 1, context=None) -> dict:
+                                         expectation=0, seed: int = 1, context=None, n_cores: int = 1,
+                                         chunked_draws: bool = False) -> dict:
     """scde.expression.difference for every contrast of `groups` (``"pairs"``, ``"rest"`` or a list of pairs; see
     ``expand_contrasts``) in one device session: ``{"<A> vs <B>": result}``."""
     with DifferenceSession(models, counts, prior, context=context) as s:
         return s.contrasts(groups, contrasts=contrasts, batch=batch, batch_models=batch_models,
                            n_randomizations=n_randomizations, return_posteriors=return_posteriors,
-                           expectation=expectation, seed=seed)
+                           expectation=expectation, seed=seed, n_cores=n_cores, chunked_draws=chunked_draws)

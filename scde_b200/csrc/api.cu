@@ -13,7 +13,9 @@
 #include <chrono>
 #include <exception>
 #include <map>
+#include <memory>
 #include <new>
+#include <atomic>
 #include <thread>
 #include <vector>
 
@@ -403,10 +405,18 @@ struct DiffWorkspace {
     DBuf<double> tbuf;                // transposition scratch for downloads
 };
 
+// The draw sets of a joint (DESIGN.md "Draw sets"): n sets of n_boot x D draws back to back, gene g using set
+// gene_set[g] (device, NULL when n == 1).  W, W8 and Z hold one block per set ([set][pass][row]); every contraction launch
+// covers all sets, each gene reading its own set's block.
+struct DrawSets {
+    int n = 1;
+    const int32_t *gene_set = nullptr;
+};
+
 // A second joint over the SAME cells (and therefore the same entry lists) with its own draws, computed in the same
 // launches of the tcgen05 kernel: the two composition-sampled joints of a batch-corrected call (R/functions.R:355-357).
 struct TwinJoint {
-    const int32_t *boot_idx_dev;  // n_boot x D
+    const int32_t *boot_idx_dev;  // n_boot x D per draw set (the first joint's sets)
     int D;
     double *jp_dev;
     JointScratch *scr;            // W, W8, Z, zpart, T, SR, spart of the second joint (the lists are the first joint's)
@@ -415,8 +425,8 @@ struct TwinJoint {
 // The tcgen05 contraction of a joint whose operands run_joint has prepared, and of its twin (NULL: none) in the same
 // launches.  The launches raise bits in *status (read_status).
 int contract_joint_i8(scde_b200_ctx *ctx, const LpTable &t, const GeneLists &lists, JointScratch &scr, int n_w_rows,
-                      int n_boot, double scale, double *jp_dev, int ld_jp, int hot_rank, int32_t *status,
-                      const TwinJoint *twin, StageTimer *tm) {
+                      int n_boot, const DrawSets &sets, double scale, double *jp_dev, int ld_jp, int hot_rank,
+                      int32_t *status, const TwinJoint *twin, StageTimer *tm) {
     cudaStream_t st = ctx->stream;
     const int passes = (n_boot + WP_TILED - 1) / WP_TILED;
     ContractI8Args q{};
@@ -428,6 +438,9 @@ int contract_joint_i8(scde_b200_ctx *ctx, const LpTable &t, const GeneLists &lis
     q.n_w_rows = n_w_rows;
     q.n_boot = n_boot;
     q.Z = scr.Z.p;
+    q.gene_set = sets.gene_set;
+    q.set_w8 = (int64_t)passes * n_w_rows * Q_WB;
+    q.set_z = (int64_t)passes * WP_TILED * KP_TILED;
     q.scale = scale;
     q.sentinel = t.sentinel;
     q.n_genes = t.n_genes;
@@ -513,8 +526,8 @@ int contract_joint_i8(scde_b200_ctx *ctx, const LpTable &t, const GeneLists &lis
 
 // The FP64 contraction of a joint whose operands run_joint has prepared (Z = NULL outside the zero-base form)
 int contract_joint_fp64(scde_b200_ctx *ctx, Contraction kernel, const LpTable &t, const GeneLists &lists,
-                        JointScratch &scr, const double *Z, int n_w_rows, int n_boot, double scale, double *jp_dev,
-                        int ld_jp, StageTimer *tm) {
+                        JointScratch &scr, const double *Z, int n_w_rows, int n_boot, const DrawSets &sets, double scale,
+                        double *jp_dev, int ld_jp, StageTimer *tm) {
     cudaStream_t st = ctx->stream;
     if (!t.f64_rows) {
         set_error("internal: the table was built in fixed point only but the FP64 contraction kernel was selected");
@@ -528,6 +541,10 @@ int contract_joint_fp64(scde_b200_ctx *ctx, Contraction kernel, const LpTable &t
     a.n_w_rows = n_w_rows;
     a.n_boot = n_boot;
     a.Z = Z;
+    const int passes = (n_boot + WP_TILED - 1) / WP_TILED;
+    a.gene_set = sets.gene_set;
+    a.set_w_rows = (int64_t)passes * n_w_rows;
+    a.set_z = (int64_t)passes * WP_TILED * t.ld;
     a.scale = scale;
     a.n_genes = t.n_genes;
     a.K = t.K;
@@ -551,20 +568,23 @@ int contract_joint_fp64(scde_b200_ctx *ctx, Contraction kernel, const LpTable &t
     return SCDE_B200_OK;
 }
 
-// jp_dev[G][ld_jp] = joint posterior of the listed cells under the draws boot_idx_dev (n_boot x D, device), on the
-// contraction kernel k selects.  The tcgen05 launches raise bits in the device word *status, which the caller has zeroed
+// jp_dev[G][ld_jp] = joint posterior of the listed cells under the draws boot_idx_dev (n_boot x D per draw set, device), on
+// the contraction kernel k selects.  The tcgen05 launches raise bits in the device word *status, which the caller has zeroed
 // (the second joint of a twin pair that did not share the launches adds to the first one's word).
 // twin (optional): see TwinJoint; only honoured on the tcgen05 path (the caller checks the return flag *twin_done and runs
 // the second joint on its own otherwise).
 int run_joint(scde_b200_ctx *ctx, ContractChoice k, const LpTable &t, const int32_t *cell_ids_dev, int n_list,
-              const int32_t *boot_idx_dev, int n_boot, int D, double scale, double *jp_dev, int ld_jp,
-              JointScratch &scr, int32_t *status, StageTimer *tm, bool count_entries, const TwinJoint *twin = nullptr,
-              bool *twin_done = nullptr) {
+              const int32_t *boot_idx_dev, int n_boot, int D, const DrawSets &sets, double scale, double *jp_dev,
+              int ld_jp, JointScratch &scr, int32_t *status, StageTimer *tm, bool count_entries,
+              const TwinJoint *twin = nullptr, bool *twin_done = nullptr) {
     cudaStream_t st = ctx->stream;
     const int n_w_rows = round_up(n_list + 1, 16);  // at least one all-zero row after the cells (list padding)
     const int passes = (n_boot + WP_TILED - 1) / WP_TILED;
     const int ld_lst = round_up(n_list, 32);
-    SCDE_CUDA(scr.W.ensure((size_t)passes * n_w_rows * WS_TILED));
+    const int S = sets.n;
+    const size_t w_set = (size_t)passes * n_w_rows * WS_TILED, z_set = (size_t)passes * WP_TILED * t.ld;
+    const size_t w8_set = (size_t)passes * n_w_rows * Q_WB, draws_set = (size_t)n_boot * D;
+    SCDE_CUDA(scr.W.ensure(S * w_set));
     SCDE_CUDA(scr.lst_row.ensure((size_t)t.n_genes * ld_lst));
     SCDE_CUDA(scr.lst_cell.ensure((size_t)t.n_genes * ld_lst));
     SCDE_CUDA(scr.lst_len.ensure((size_t)t.n_genes));
@@ -572,11 +592,12 @@ int run_joint(scde_b200_ctx *ctx, ContractChoice k, const LpTable &t, const int3
     SCDE_CUDA(scr.total.ensure(1));
     const bool zb = t.zero_base && t.ld <= KP_TILED;
     if (zb) {
-        SCDE_CUDA(scr.Z.ensure((size_t)passes * WP_TILED * t.ld));
+        SCDE_CUDA(scr.Z.ensure(S * z_set));
         SCDE_CUDA(scr.zpart.ensure(base_sum_scratch_doubles(n_boot, t.ld)));
     }
     const int e0 = tm ? tm->begin(st) : -1;
-    SCDE_CUDA(launch_build_w(boot_idx_dev, n_boot, D, n_list, scr.W.p, n_w_rows, st));
+    for (int s = 0; s < S; ++s)
+        SCDE_CUDA(launch_build_w(boot_idx_dev + s * draws_set, n_boot, D, n_list, scr.W.p + s * w_set, n_w_rows, st));
     SCDE_CUDA(cudaMemsetAsync(jp_dev, 0, sizeof(double) * (size_t)t.n_genes * ld_jp, st));
     GeneLists lists{scr.lst_row.p, scr.lst_cell.p, scr.lst_len.p, scr.order.p, ld_lst};
     const bool i8 = zb && t.has_q && k.kernel == Contraction::I8 && contract_i8_supported(t.K, t.ld, ld_lst, D);
@@ -591,29 +612,36 @@ int run_joint(scde_b200_ctx *ctx, ContractChoice k, const LpTable &t, const int3
                                  zb ? t.based.p : nullptr, 0, lists, count_entries ? scr.total.p : nullptr, st, hot_rank,
                                  tw ? 2 : 1));
     if (zb)
-        SCDE_CUDA(launch_base_sum(t.table.p, t.ld, t.zero_row.p, t.based.p, cell_ids_dev, n_list, scr.W.p, n_w_rows, n_boot,
-                                  scr.Z.p, scr.zpart.p, st, t.zero_compact));
+        for (int s = 0; s < S; ++s)
+            SCDE_CUDA(launch_base_sum(t.table.p, t.ld, t.zero_row.p, t.based.p, cell_ids_dev, n_list, scr.W.p + s * w_set,
+                                      n_w_rows, n_boot, scr.Z.p + s * z_set, scr.zpart.p, st, t.zero_compact));
+    // W8 of all sets in one conversion: the sets' blocks are consecutive rows
     if (tw) {  // the second joint's W, base sums and output
         JointScratch &s2 = *twin->scr;
-        SCDE_CUDA(s2.W.ensure((size_t)passes * n_w_rows * WS_TILED));
-        SCDE_CUDA(s2.Z.ensure((size_t)passes * WP_TILED * t.ld));
+        const size_t twin_draws_set = (size_t)n_boot * twin->D;
+        SCDE_CUDA(s2.W.ensure(S * w_set));
+        SCDE_CUDA(s2.Z.ensure(S * z_set));
         SCDE_CUDA(s2.zpart.ensure(base_sum_scratch_doubles(n_boot, t.ld)));
-        SCDE_CUDA(s2.W8.ensure((size_t)passes * n_w_rows * Q_WB));
-        SCDE_CUDA(launch_build_w(twin->boot_idx_dev, n_boot, twin->D, n_list, s2.W.p, n_w_rows, st));
+        SCDE_CUDA(s2.W8.ensure(S * w8_set));
+        for (int s = 0; s < S; ++s)
+            SCDE_CUDA(launch_build_w(twin->boot_idx_dev + s * twin_draws_set, n_boot, twin->D, n_list, s2.W.p + s * w_set,
+                                     n_w_rows, st));
         SCDE_CUDA(cudaMemsetAsync(twin->jp_dev, 0, sizeof(double) * (size_t)t.n_genes * ld_jp, st));
-        SCDE_CUDA(launch_base_sum(t.table.p, t.ld, t.zero_row.p, t.based.p, cell_ids_dev, n_list, s2.W.p, n_w_rows, n_boot,
-                                  s2.Z.p, s2.zpart.p, st, t.zero_compact));
-        SCDE_CUDA(launch_w_to_i8(s2.W.p, n_w_rows, n_boot, s2.W8.p, status, st));
+        for (int s = 0; s < S; ++s)
+            SCDE_CUDA(launch_base_sum(t.table.p, t.ld, t.zero_row.p, t.based.p, cell_ids_dev, n_list, s2.W.p + s * w_set,
+                                      n_w_rows, n_boot, s2.Z.p + s * z_set, s2.zpart.p, st, t.zero_compact));
+        SCDE_CUDA(launch_w_to_i8(s2.W.p, S * n_w_rows, n_boot, s2.W8.p, status, st));
     }
     if (i8) {
-        SCDE_CUDA(scr.W8.ensure((size_t)passes * n_w_rows * Q_WB));
-        SCDE_CUDA(launch_w_to_i8(scr.W.p, n_w_rows, n_boot, scr.W8.p, status, st));
+        SCDE_CUDA(scr.W8.ensure(S * w8_set));
+        SCDE_CUDA(launch_w_to_i8(scr.W.p, S * n_w_rows, n_boot, scr.W8.p, status, st));
     }
-    if (tm) tm->end(SCDE_B200_T_OTHER, e0, st, (zb ? 5 : 3) + (i8 ? 1 : 0) + (tw ? 5 : 0));
+    // build_w is a memset and a kernel, base_sum two kernels: per extra set
+    if (tm) tm->end(SCDE_B200_T_OTHER, e0, st, (zb ? 5 : 3) + (i8 ? 1 : 0) + (tw ? 5 : 0) + (S - 1) * ((zb ? 4 : 2) + (tw ? 4 : 0)));
     if (!i8)
-        return contract_joint_fp64(ctx, k.kernel, t, lists, scr, zb ? scr.Z.p : nullptr, n_w_rows, n_boot, scale, jp_dev,
-                                   ld_jp, tm);
-    return contract_joint_i8(ctx, t, lists, scr, n_w_rows, n_boot, scale, jp_dev, ld_jp, hot_rank, status,
+        return contract_joint_fp64(ctx, k.kernel, t, lists, scr, zb ? scr.Z.p : nullptr, n_w_rows, n_boot, sets, scale,
+                                   jp_dev, ld_jp, tm);
+    return contract_joint_i8(ctx, t, lists, scr, n_w_rows, n_boot, sets, scale, jp_dev, ld_jp, hot_rank, status,
                              tw ? twin : nullptr, tm);
 }
 
@@ -852,6 +880,108 @@ void shard_range(int N, int n, int i, int *b, int *e) {
     const int base = N / n, rem = N % n;
     *b = i * base + (i < rem ? i : rem);
     *e = *b + base + (i < rem ? 1 : 0);
+}
+
+// The draw sets a call or shard over genes [g0, g1) of N holds (DESIGN.md "Draw sets"): the reference's n.cores = n splits
+// [0, N) into n chunks (shard_range, R/functions.R:606-617) when n > 1 and N > n, and chunk i = [b_i, e_i) draws with
+// Seed = seed + b_i; otherwise one set from `seed`.  The sets are the chunks that meet [g0, g1), in order.
+struct DrawChunks {
+    int first = 0;                  // global index of the first set's chunk
+    std::vector<int32_t> seeds;     // one per set
+    std::vector<int32_t> gene_set;  // per gene of [g0, g1): its set; empty with one set
+    int n_sets() const { return (int)seeds.size(); }
+};
+
+int check_draw_chunks(int32_t n, bool explicit_draws, const char *who) {
+    if (n < 0) {
+        set_error("%s: draw_chunks %d < 0", who, n);
+        return SCDE_B200_EINVAL;
+    }
+    if (n > SCDE_B200_MAX_DRAW_CHUNKS) {
+        set_error("%s: draw_chunks %d above SCDE_B200_MAX_DRAW_CHUNKS (%d)", who, n, SCDE_B200_MAX_DRAW_CHUNKS);
+        return SCDE_B200_ELIMIT;
+    }
+    if (n > 1 && explicit_draws) {
+        set_error("%s: draw_chunks > 1 draws every gene chunk from its own seed; it cannot be combined with explicit boot_idx",
+                  who);
+        return SCDE_B200_EINVAL;
+    }
+    return SCDE_B200_OK;
+}
+
+// the seeds of all draw sets over genes [0, N), in chunk order
+std::vector<int32_t> chunk_seeds(int N, int n, int seed) {
+    if (!(n > 1 && N > n)) return {seed};
+    std::vector<int32_t> v(n);
+    for (int i = 0; i < n; ++i) {
+        int b = 0, e = 0;
+        shard_range(N, n, i, &b, &e);
+        v[i] = seed + b;
+    }
+    return v;
+}
+
+DrawChunks draw_chunks_of(int N, int n, int seed, int g0, int g1) {
+    DrawChunks d;
+    if (!(n > 1 && N > n)) {
+        d.seeds.push_back(seed);
+        return d;
+    }
+    for (int i = 0; i < n; ++i) {
+        int b = 0, e = 0;
+        shard_range(N, n, i, &b, &e);
+        if (e <= g0 || b >= g1) continue;
+        if (d.seeds.empty()) d.first = i;
+        const int set = d.n_sets();
+        d.seeds.push_back(seed + b);
+        for (int g = b > g0 ? b : g0; g < (e < g1 ? e : g1); ++g) d.gene_set.push_back(set);
+    }
+    if (d.n_sets() == 1) d.gene_set.clear();
+    return d;
+}
+
+// Helper threads of parallel_for alive in the process.  Concurrent calls (one per device shard of a multi-device context)
+// share one budget of hardware_concurrency() - 1 helpers, so they never oversubscribe the host together.
+std::atomic<int> g_helper_threads{0};
+
+// Runs f(i) for i < n on the calling thread plus as many helper threads as the process-wide budget allows (none when
+// n <= 1 or the budget is spent: the calling thread then runs every task); f returns a status, the first failure (in
+// task order) is returned.  A helper thread that cannot be started is simply not used.  The draw sets of a call are
+// independent: they are generated in parallel.
+template <class F>
+int parallel_for(int n, F f) {
+    if (n <= 0) return SCDE_B200_OK;
+    if (n == 1) return f(0);
+    std::atomic<int> next{0};
+    std::vector<int> rc(n, SCDE_B200_OK);
+    std::vector<std::string> msg(n);
+    auto worker = [&] {
+        for (int i; (i = next.fetch_add(1)) < n;)
+            if ((rc[i] = f(i)) != SCDE_B200_OK) msg[i] = g_err;  // the error text is thread-local
+    };
+    const int hw = std::thread::hardware_concurrency() > 0 ? (int)std::thread::hardware_concurrency() : 1;
+    const int want = (n < hw ? n : hw) - 1;
+    int reserved = 0;
+    while (reserved < want) {
+        int cur = g_helper_threads.load();
+        if (cur >= hw - 1) break;
+        if (g_helper_threads.compare_exchange_weak(cur, cur + 1)) ++reserved;
+    }
+    std::vector<std::thread> th;
+    try {
+        th.reserve(reserved);
+        for (int i = 0; i < reserved; ++i) th.emplace_back(worker);
+    } catch (...) {  // no further helpers: the started ones and the calling thread share the tasks
+    }
+    worker();
+    for (auto &t : th) t.join();
+    g_helper_threads.fetch_sub(reserved);
+    for (int i = 0; i < n; ++i)
+        if (rc[i] != SCDE_B200_OK) {
+            g_err = msg[i];
+            return rc[i];
+        }
+    return SCDE_B200_OK;
 }
 
 // Runs f(i) for i < n on one host thread each (directly when n == 1); exceptions become return codes, the first failing
@@ -1261,7 +1391,7 @@ static int log_boot_impl(scde_b200_ctx *ctx, const double *models, int32_t n_cel
         }
         TRY(validate_index(boot_idx, (size_t)nb * dd, 0, n_cells, "boot_idx"));
         TRY(upload(d_boot, boot_idx, (size_t)nb * dd, st));
-        TRY(run_joint(ctx, k, t, nullptr, n_cells, d_boot.p, nb, dd, scale, d_jp.p, ld_jp, scr, status.p, nullptr, false));
+        TRY(run_joint(ctx, k, t, nullptr, n_cells, d_boot.p, nb, dd, {}, scale, d_jp.p, ld_jp, scr, status.p, nullptr, false));
     }
     SCDE_CUDA(d_out.ensure((size_t)n_genes * n_grid));
     SCDE_CUDA(launch_transpose_out(d_jp.p, ld_jp, n_genes, n_grid, d_out.p, st));
@@ -1398,7 +1528,7 @@ static int jpmat_common(scde_b200_ctx *ctx, const double *matl, int n_mat, int n
     JointScratch scr;
     if (n_boot > 0) {
         // not divided by n_boot: src/jpmatLogBoot.cpp:36-38 (no fixed-point table: no tcgen05 launch, no status word)
-        TRY(run_joint(ctx, contraction_choice(ctx), t, nullptr, n_mat, d_boot.p, n_boot, D, 1.0, d_jp.p, t.ld, scr, nullptr,
+        TRY(run_joint(ctx, contraction_choice(ctx), t, nullptr, n_mat, d_boot.p, n_boot, D, {}, 1.0, d_jp.p, t.ld, scr, nullptr,
                       nullptr, false));
     } else {
         SCDE_CUDA(cudaMemsetAsync(d_jp.p, 0, sizeof(double) * (size_t)n_rows * t.ld, st));
@@ -1787,8 +1917,10 @@ struct scde_b200_diff_job {
     ModelSet bmodels;           // batch.models when they differ from models (else empty)
     DBuf<double> mag, prior_y;
     DBuf<int32_t> cell_ids[2];  // group cell lists
-    DBuf<int32_t> boot[4];
+    DBuf<int32_t> boot[4];      // draws of each joint: one block of n_boot x D[i] per draw set
     int D[4] = {0, 0, 0, 0};
+    DrawChunks chunks;          // the draw sets of the job's genes
+    DBuf<int32_t> gene_set;     // chunks.gene_set on the device
     DBuf<int32_t> zi, zi_adj;
     DBuf<int32_t> idx, bidx, aidx;
     DBuf<double> z, bz, az;
@@ -1806,7 +1938,7 @@ struct scde_b200_diff_job {
     TablePlan front_plan;            // the front's table plan (buffers bound in its first phase)
     const int32_t *boot_ptr[4] = {nullptr, nullptr, nullptr, nullptr};  // draws as the device reads them
     std::vector<int32_t> ids[2];                 // cells of the two groups
-    std::vector<int32_t> gen[4];                 // generated draws, alive until their uploads have completed
+    std::unique_ptr<int32_t[]> gen[4];           // generated draws (resident job), alive until their uploads have completed
     const scde_b200_diff_args *deferred_args = nullptr;  // one-shot call: the draws are still to be generated and uploaded
 };
 
@@ -1818,40 +1950,29 @@ struct scde_b200_diff_job {
 int upload_draws(scde_b200_ctx *ctx, scde_b200_diff_job *j, const scde_b200_diff_args *a, bool pinned = false) {
     cudaStream_t st = ctx->stream;
     const int C = j->C;
-    const int32_t *src[4] = {nullptr, nullptr, nullptr, nullptr};
-    // host work first (the uploads below may wait for the kernels already queued on the stream)
-    for (int i = 0; i < 2; ++i) {
-        const int n = j->n_group[i];
-        src[i] = a->boot_idx[i];
-        if (!src[i]) {
-            j->gen[i] = gen_boot(a->seed, n, a->n_boot);
-            src[i] = j->gen[i].data();
-        }
-        TRY(validate_index(src[i], (size_t)a->n_boot * n, 0, n, "boot_idx"));
-        j->D[i] = n;
-    }
+    const int S = j->chunks.n_sets();  // draw sets per joint (a->boot_idx are NULL when S > 1)
+    const int n_joints = j->has_batch ? 4 : 2;
+    // draws per joint and the caller's explicit draws, validated
+    BatchPools bp;
+    std::vector<int32_t> comp[2];
+    for (int i = 0; i < 2; ++i) j->D[i] = j->n_group[i];
     if (j->has_batch) {
-        const int L = a->n_batch_levels;
-        BatchPools bp;
-        TRY(batch_pools(a->batch, C, L, bp));
-        for (int i = 0; i < 2; ++i) {
-            std::vector<int32_t> comp;
-            const int D = batch_composition(a->batch, L, j->ids[i].data(), j->ids[i].size(), comp);
-            src[2 + i] = a->boot_idx[2 + i];
-            if (!src[2 + i]) {
-                j->gen[2 + i].resize((size_t)a->n_boot * D);
-                TRY(scde_b200_batch_boot_indices(a->seed, L, bp.off.data(), bp.pool.data(), comp.data(), a->n_boot,
-                                                 j->gen[2 + i].data()));
-                src[2 + i] = j->gen[2 + i].data();
-            }
-            if (D > 0) TRY(validate_index(src[2 + i], (size_t)a->n_boot * D, 0, C, "batch boot_idx"));
-            j->D[2 + i] = D;
-        }
+        TRY(batch_pools(a->batch, C, a->n_batch_levels, bp));
+        for (int i = 0; i < 2; ++i)
+            j->D[2 + i] = batch_composition(a->batch, a->n_batch_levels, j->ids[i].data(), j->ids[i].size(), comp[i]);
     }
-    const int n_sets = j->has_batch ? 4 : 2;
+    for (int i = 0; i < n_joints; ++i)
+        if (a->boot_idx[i] && j->D[i] > 0)
+            TRY(validate_index(a->boot_idx[i], (size_t)a->n_boot * j->D[i], 0, i < 2 ? j->D[i] : C,
+                               i < 2 ? "boot_idx" : "batch boot_idx"));
+    // Destinations: the mapped pinned staging (read in place by the W build) or, for an upload, host buffers that are
+    // not zero-filled first.  The generators write straight into them, one (joint, set) per task on parallel host
+    // threads, so the one-shot call pays neither a zero-fill nor a copy of the draws before its first joint.
+    int32_t *dst[4] = {nullptr, nullptr, nullptr, nullptr};
+    int32_t *dev = nullptr;
     if (pinned) {
         size_t total = 0;
-        for (int i = 0; i < n_sets; ++i) total += (size_t)a->n_boot * j->D[i];
+        for (int i = 0; i < n_joints; ++i) total += (size_t)S * a->n_boot * j->D[i];
         if (total > ctx->h_draws_cap) {
             if (ctx->h_draws) cudaFreeHost(ctx->h_draws);
             ctx->h_draws = nullptr;
@@ -1859,19 +1980,44 @@ int upload_draws(scde_b200_ctx *ctx, scde_b200_diff_job *j, const scde_b200_diff
             SCDE_CUDA(cudaHostAlloc((void **)&ctx->h_draws, sizeof(int32_t) * total, cudaHostAllocMapped));
             ctx->h_draws_cap = total;
         }
-        int32_t *dev = nullptr;
         SCDE_CUDA(cudaHostGetDevicePointer((void **)&dev, ctx->h_draws, 0));
         size_t off = 0;
-        for (int i = 0; i < n_sets; ++i) {
-            const size_t n = (size_t)a->n_boot * j->D[i];
-            memcpy(ctx->h_draws + off, src[i], sizeof(int32_t) * n);
+        for (int i = 0; i < n_joints; ++i) {
+            dst[i] = ctx->h_draws + off;
             j->boot_ptr[i] = dev + off;
-            off += n;
+            off += (size_t)S * a->n_boot * j->D[i];
         }
-        return SCDE_B200_OK;
+    } else {
+        for (int i = 0; i < n_joints; ++i)
+            if (!a->boot_idx[i]) {
+                j->gen[i].reset(new int32_t[(size_t)S * a->n_boot * j->D[i]]);
+                dst[i] = j->gen[i].get();
+            }
     }
-    for (int i = 0; i < n_sets; ++i) {
-        TRY(upload(j->boot[i], src[i], (size_t)a->n_boot * j->D[i], st));
+    std::vector<std::pair<int, int>> tasks;  // (joint, set); an explicit set is one copy task (pinned) or none
+    for (int i = 0; i < n_joints; ++i) {
+        if (a->boot_idx[i]) {
+            if (pinned) tasks.emplace_back(i, -1);
+            continue;
+        }
+        for (int s = 0; s < S; ++s) tasks.emplace_back(i, s);
+    }
+    const std::vector<int32_t> &seeds = j->chunks.seeds;
+    TRY(parallel_for((int)tasks.size(), [&](int t) -> int {
+        const int i = tasks[t].first, s = tasks[t].second;
+        const size_t per = (size_t)a->n_boot * j->D[i];
+        if (s < 0) {
+            memcpy(dst[i], a->boot_idx[i], sizeof(int32_t) * per);
+            return SCDE_B200_OK;
+        }
+        int32_t *out = dst[i] + s * per;
+        if (i < 2) return scde_b200_boot_indices(seeds[s], j->n_group[i], a->n_boot, out);
+        return scde_b200_batch_boot_indices(seeds[s], a->n_batch_levels, bp.off.data(), bp.pool.data(), comp[i - 2].data(),
+                                            a->n_boot, out);
+    }));
+    if (pinned) return SCDE_B200_OK;
+    for (int i = 0; i < n_joints; ++i) {
+        TRY(upload(j->boot[i], a->boot_idx[i] ? a->boot_idx[i] : dst[i], (size_t)S * a->n_boot * j->D[i], st));
         j->boot_ptr[i] = j->boot[i].p;
     }
     SCDE_CUDA(cudaStreamSynchronize(st));  // the caller's (or the job's) host arrays have been read
@@ -1985,6 +2131,8 @@ static int diff_upload_impl(scde_b200_ctx *ctx, ContractChoice k, const scde_b20
     }
     int g0 = 0, g1 = 0;
     TRY(gene_range(a, &g0, &g1));
+    TRY(check_draw_chunks(a->draw_chunks, a->boot_idx[0] || a->boot_idx[1] || a->boot_idx[2] || a->boot_idx[3],
+                          "expression_difference"));
     const int G = g1 - g0, C = a->n_cells, K = a->n_grid;
     std::vector<int32_t> ids[2];
     for (int c = 0; c < C; ++c)
@@ -2060,6 +2208,8 @@ static int diff_upload_impl(scde_b200_ctx *ctx, ContractChoice k, const scde_b20
     // kernels run (upload_draws is then called by diff_run_impl)
     j->ids[0] = ids[0];
     j->ids[1] = ids[1];
+    j->chunks = draw_chunks_of(a->n_genes, a->draw_chunks, a->seed, g0, g1);
+    if (j->chunks.n_sets() > 1) JTRY(upload(j->gene_set, j->chunks.gene_set.data(), j->chunks.gene_set.size(), st));
     if (defer_counts)
         j->deferred_args = a;
     else
@@ -2263,8 +2413,9 @@ static int diff_run_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, bool chunked
     SCDE_CUDA(cudaMemsetAsync(j->status.p, 0, 3 * sizeof(int32_t), st));
     int t_all = tm.begin(st);
     bool front_done = false, joint0_done = false;
+    const DrawSets sets{j->chunks.n_sets(), j->gene_set.p};
     auto group_joint = [&](int i) {  // cells of one factor level, draws are local indices (R/functions.R:372-374)
-        return run_joint(ctx, k, j->ws->table, j->cell_ids[i].p, j->n_group[i], j->boot_ptr[i], j->n_boot, j->D[i],
+        return run_joint(ctx, k, j->ws->table, j->cell_ids[i].p, j->n_group[i], j->boot_ptr[i], j->n_boot, j->D[i], sets,
                          (double)j->n_boot, j->ws->jp[i].p, ld, j->ws->scr, j->status.p + i, &tm, true);
     };
     if (chunked_counts) {
@@ -2306,10 +2457,10 @@ static int diff_run_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, bool chunked
         // kernel for both, items paired on neighbouring SMs, so the table is pulled from DRAM once for the two
         TwinJoint tw{j->boot_ptr[3], j->D[3], j->ws->jp[3].p, &j->ws->scr2};
         bool twin_done = false;
-        TRY(run_joint(ctx, k, j->ws->table, nullptr, C, j->boot_ptr[2], j->n_boot, j->D[2], (double)j->n_boot, j->ws->jp[2].p,
-                      ld, j->ws->scr, j->status.p + 2, &tm, true, &tw, &twin_done));
+        TRY(run_joint(ctx, k, j->ws->table, nullptr, C, j->boot_ptr[2], j->n_boot, j->D[2], sets, (double)j->n_boot,
+                      j->ws->jp[2].p, ld, j->ws->scr, j->status.p + 2, &tm, true, &tw, &twin_done));
         if (!twin_done)
-            TRY(run_joint(ctx, k, j->ws->table, nullptr, C, j->boot_ptr[3], j->n_boot, j->D[3], (double)j->n_boot,
+            TRY(run_joint(ctx, k, j->ws->table, nullptr, C, j->boot_ptr[3], j->n_boot, j->D[3], sets, (double)j->n_boot,
                           j->ws->jp[3].p, ld, j->ws->scr, j->status.p + 2, &tm, true));
     }
     const int e0 = tm.begin(st);
@@ -2469,10 +2620,10 @@ int scde_b200_expression_difference(scde_b200_ctx *ctx, const scde_b200_diff_arg
     }
     int g0 = 0, g1 = 0;
     TRY(gene_range(args, &g0, &g1));
-    // Several devices: contiguous gene ranges, one per device (the split the reference's chunk() makes for n.cores,
-    // R/functions.R:606), every shard with the same Seed and therefore the same draws -- the n.cores = 1 semantics, so the
-    // result does not depend on the number of devices.  No inter-GPU traffic: every shard's results go to its rows of the
-    // caller's buffers by device-to-host copies.
+    // Several devices: contiguous gene ranges, one per device.  Every shard holds the draw sets of the draw chunks it
+    // meets, with their global seeds (draw_chunks_of over the call's n_genes), so the result does not depend on the number
+    // of devices.  No inter-GPU traffic: every shard's results go to its rows of the caller's buffers by device-to-host
+    // copies.
     const std::vector<scde_b200_ctx *> devs = context_devices(ctx);
     const int n = g1 - g0;
     const int n_use = (int)devs.size() < n ? (int)devs.size() : n;
@@ -2509,10 +2660,12 @@ struct ContrastPlan {
     std::vector<int> slot_group;      // bank slot -> group id (only groups some contrast names)
     std::vector<int32_t> cells;       // the slots' cells back to back
     std::vector<int64_t> cell_off;    // slot -> offset into cells (n_slots + 1)
-    std::vector<int32_t> draws;       // group draws, one set per distinct group size
+    int seed = 1, draw_chunks = 0;    // the draw sets: DrawChunks over the dataset's genes
+    int n_sets = 1;                   // draw sets over all genes (a shard uses those of the chunks it meets)
+    std::vector<int32_t> draws;       // group draws per distinct group size: n_sets blocks of n_boot x size
     std::vector<int64_t> draw_off;    // slot -> offset into draws
     std::vector<int> bslot_D;         // batch slot (distinct composition) -> draws per boot
-    std::vector<int32_t> bdraws;      // batch draws (global cell ids), one set per batch slot
+    std::vector<int32_t> bdraws;      // batch draws (global cell ids) per batch slot: n_sets blocks of n_boot x D
     std::vector<int64_t> bdraw_off;
     std::vector<int> pair_slot, pair_bslot;  // 2 per contrast
     std::vector<int32_t> zi, zi_adj;  // n_zero entries each (1 or N)
@@ -2535,7 +2688,7 @@ struct DatasetShard {
     int rows_from = 0;
     bool rows_i8 = false;
     DBuf<double> bank, bbank;                 // joint posteriors, [slot][G][ld]
-    DBuf<int32_t> cells, draws, bdraws, zi, zi_adj, jflags;
+    DBuf<int32_t> cells, draws, bdraws, zi, zi_adj, jflags, gene_set;
     DBuf<int32_t> idx, bidx, aidx;            // [contrast][3][G]
     DBuf<double> z, bz, az;                   // [contrast][G]
     DBuf<RatioContrast> rtab;                 // [pass][contrast] device tables of the batched ratio launches
@@ -2635,8 +2788,44 @@ int shard_contrasts(DatasetShard &sh, const ContrastPlan &p, const scde_b200_con
     const int t_all = tm.begin(st);
     TRY(ensure_rows(sh, 0, k, &tm));
     TRY(upload(sh.cells, p.cells.data(), p.cells.size(), st));
-    TRY(upload(sh.draws, p.draws.data(), p.draws.size(), st));
-    if (p.has_batch) TRY(upload(sh.bdraws, p.bdraws.data(), p.bdraws.size(), st));
+    // this shard's draw sets: those of the chunks it meets.  Only they are uploaded, packed per group size (and per batch
+    // composition); sh_draw_off / sh_bdraw_off map a plan offset (the block of all sets) to the packed block on the device.
+    const DrawChunks dc = draw_chunks_of(p.N, p.draw_chunks, p.seed, sh.g0, sh.g0 + G);
+    std::map<int64_t, int64_t> sh_draw_off;
+    std::vector<int64_t> sh_bdraw_off(p.bdraw_off.size());
+    {
+        auto pack = [&](DBuf<int32_t> &buf, const std::vector<int32_t> &all, const std::vector<std::pair<int64_t, int64_t>> &blocks,
+                        std::vector<int64_t> &local) -> int {  // blocks: (plan offset, draws per set)
+            int64_t total = 0;
+            for (const auto &b : blocks) total += (int64_t)dc.n_sets() * b.second;
+            SCDE_CUDA(buf.ensure((size_t)(total > 0 ? total : 1)));
+            int64_t off = 0;
+            local.clear();
+            for (const auto &b : blocks) {
+                local.push_back(off);
+                const int64_t n = (int64_t)dc.n_sets() * b.second;
+                if (n > 0)
+                    SCDE_CUDA(cudaMemcpyAsync(buf.p + off, all.data() + b.first + (int64_t)dc.first * b.second,
+                                              sizeof(int32_t) * n, cudaMemcpyHostToDevice, st));
+                off += n;
+            }
+            return SCDE_B200_OK;
+        };
+        std::vector<std::pair<int64_t, int64_t>> blocks;
+        for (int s = 0; s < n_slots; ++s)
+            if (!sh_draw_off.count(p.draw_off[s])) {
+                sh_draw_off[p.draw_off[s]] = -1;
+                blocks.emplace_back(p.draw_off[s], (int64_t)p.n_boot * (p.cell_off[s + 1] - p.cell_off[s]));
+            }
+        std::vector<int64_t> local;
+        TRY(pack(sh.draws, p.draws, blocks, local));
+        for (size_t i = 0; i < blocks.size(); ++i) sh_draw_off[blocks[i].first] = local[i];
+        if (p.has_batch) {
+            blocks.clear();
+            for (int b = 0; b < n_bslots; ++b) blocks.emplace_back(p.bdraw_off[b], (int64_t)p.n_boot * p.bslot_D[b]);
+            TRY(pack(sh.bdraws, p.bdraws, blocks, sh_bdraw_off));
+        }
+    }
     {
         const std::vector<int32_t> zi = zero_slice(p.zi.data(), p.n_zero, sh.g0, G);
         TRY(upload(sh.zi, zi.data(), zi.size(), st));
@@ -2655,13 +2844,20 @@ int shard_contrasts(DatasetShard &sh, const ContrastPlan &p, const scde_b200_con
     const int n_words = n_slots + (n_bslots + 1) / 2;
     SCDE_CUDA(sh.jflags.ensure((size_t)n_words));
     SCDE_CUDA(cudaMemsetAsync(sh.jflags.p, 0, sizeof(int32_t) * n_words, st));
+    if (dc.n_sets() > 1) {
+        TRY(upload(sh.gene_set, dc.gene_set.data(), dc.gene_set.size(), st));
+        SCDE_CUDA(cudaStreamSynchronize(st));
+    }
+    const DrawSets sets{dc.n_sets(), dc.n_sets() > 1 ? sh.gene_set.p : nullptr};
+    auto group_draws = [&](int s) { return sh.draws.p + sh_draw_off.at(p.draw_off[s]); };
+    auto batch_draws = [&](int b) { return sh.bdraws.p + sh_bdraw_off[b]; };
     auto group_joint = [&](int s, ContractChoice kk, bool count) {
         const int n = (int)(p.cell_off[s + 1] - p.cell_off[s]);
-        return run_joint(ctx, kk, t, sh.cells.p + p.cell_off[s], n, sh.draws.p + p.draw_off[s], p.n_boot, n, (double)p.n_boot,
+        return run_joint(ctx, kk, t, sh.cells.p + p.cell_off[s], n, group_draws(s), p.n_boot, n, sets, (double)p.n_boot,
                          sh.bank.p + s * slot_sz, ld, ws->scr, sh.jflags.p + s, &tm, count);
     };
     auto batch_joint = [&](int b, ContractChoice kk, bool count, const TwinJoint *tw, bool *twin_done) {
-        return run_joint(ctx, kk, t, nullptr, sh.C, sh.bdraws.p + p.bdraw_off[b], p.n_boot, p.bslot_D[b], (double)p.n_boot,
+        return run_joint(ctx, kk, t, nullptr, sh.C, batch_draws(b), p.n_boot, p.bslot_D[b], sets, (double)p.n_boot,
                          sh.bbank.p + b * slot_sz, ld, ws->scr, sh.jflags.p + n_slots + b / 2, &tm, count, tw, twin_done);
     };
     for (int s = 0; s < n_slots; ++s) TRY(group_joint(s, k, true));
@@ -2671,7 +2867,7 @@ int shard_contrasts(DatasetShard &sh, const ContrastPlan &p, const scde_b200_con
         for (int b = 0; b < n_bslots; b += 2) {
             bool twin_done = false;
             if (b + 1 < n_bslots) {
-                TwinJoint tw{sh.bdraws.p + p.bdraw_off[b + 1], p.bslot_D[b + 1], sh.bbank.p + (b + 1) * slot_sz, &ws->scr2};
+                TwinJoint tw{batch_draws(b + 1), p.bslot_D[b + 1], sh.bbank.p + (b + 1) * slot_sz, &ws->scr2};
                 TRY(batch_joint(b, k, true, &tw, &twin_done));
                 if (!twin_done) TRY(batch_joint(b + 1, k, true, nullptr, nullptr));
             } else {
@@ -2796,6 +2992,7 @@ int plan_contrasts(const scde_b200_dataset *ds, const scde_b200_contrast_args *a
     if (a->n_groups < 2 || !a->group_offsets || !a->group_cells) return bad("contrasts: need at least two groups");
     if (a->n_contrasts < 1 || !a->pairs) return bad("contrasts: need at least one contrast");
     if (a->n_boot < 1) return bad("contrasts: n_boot must be >= 1");
+    TRY(check_draw_chunks(a->draw_chunks, false, "contrasts"));
     if ((o->cz && !o->z) || (o->batch_cz && !o->batch_z) || (o->adjusted_cz && !o->adjusted_z))
         return bad("contrasts: a cZ output needs the matching Z output");
     if (a->group_offsets[0] != 0) return bad("contrasts: group_offsets[0] must be 0");
@@ -2826,6 +3023,10 @@ int plan_contrasts(const scde_b200_dataset *ds, const scde_b200_contrast_args *a
     p.n_zero = a->n_zero;
     p.n_contrasts = a->n_contrasts;
     p.n_boot = a->n_boot;
+    p.seed = a->seed;
+    p.draw_chunks = a->draw_chunks;
+    const std::vector<int32_t> seeds = chunk_seeds(N, a->draw_chunks, a->seed);
+    p.n_sets = (int)seeds.size();
     p.want_post = o->difference_posterior || o->adjusted_difference_posterior;
     std::vector<int> slot_of(a->n_groups, -1);
     p.pair_slot.resize(2 * (size_t)a->n_contrasts);
@@ -2851,6 +3052,9 @@ int plan_contrasts(const scde_b200_dataset *ds, const scde_b200_contrast_args *a
         }
     }
     // group joints: cells of every slot, draws once per distinct group size (local indices, src/jpmatLogBoot.cpp:221,254-257)
+    // and draw set; the draws are generated below, on parallel host threads, one (size or composition, set) each
+    const int S = p.n_sets;
+    std::vector<std::pair<int64_t, int>> group_tasks;  // (offset of the set's block, size)
     std::map<int, int64_t> draws_of_size;
     p.cell_off.assign(1, 0);
     for (int g : p.slot_group) {
@@ -2861,15 +3065,20 @@ int plan_contrasts(const scde_b200_dataset *ds, const scde_b200_contrast_args *a
         auto it = draws_of_size.find(n);
         if (it == draws_of_size.end()) {
             it = draws_of_size.emplace(n, (int64_t)p.draws.size()).first;
-            const std::vector<int32_t> d = gen_boot(a->seed, n, a->n_boot);
-            p.draws.insert(p.draws.end(), d.begin(), d.end());
+            for (int s = 0; s < S; ++s) group_tasks.emplace_back(it->second + (int64_t)s * a->n_boot * n, n);
+            p.draws.resize(p.draws.size() + (size_t)S * a->n_boot * n);
         }
         p.draw_off.push_back(it->second);
     }
+    TRY(parallel_for((int)group_tasks.size(), [&](int i) -> int {
+        const auto &tk = group_tasks[i];
+        return scde_b200_boot_indices(seeds[(size_t)i % S], tk.second, a->n_boot, p.draws.data() + tk.first);
+    }));
     if (!p.has_batch) return SCDE_B200_OK;
     // batch joints: one per distinct composition table(batch[group]) (R/functions.R:355-357)
     const int L = a->n_batch_levels;
     std::map<std::vector<int32_t>, int> bslot_of;
+    std::vector<std::vector<int32_t>> bcomp;  // composition of every batch slot
     std::vector<int> bslot_of_slot(p.slot_group.size());
     for (size_t s = 0; s < p.slot_group.size(); ++s) {
         std::vector<int32_t> comp;
@@ -2880,12 +3089,16 @@ int plan_contrasts(const scde_b200_dataset *ds, const scde_b200_contrast_args *a
             it = bslot_of.emplace(comp, (int)p.bslot_D.size()).first;
             p.bslot_D.push_back(D);
             p.bdraw_off.push_back((int64_t)p.bdraws.size());
-            p.bdraws.resize(p.bdraws.size() + (size_t)a->n_boot * D);
-            TRY(scde_b200_batch_boot_indices(a->seed, L, bp.off.data(), bp.pool.data(), comp.data(), a->n_boot,
-                                             p.bdraws.data() + p.bdraw_off.back()));
+            p.bdraws.resize(p.bdraws.size() + (size_t)S * a->n_boot * D);
+            bcomp.push_back(comp);
         }
         bslot_of_slot[s] = it->second;
     }
+    TRY(parallel_for((int)bcomp.size() * S, [&](int i) -> int {
+        const int b = i / S, set = i % S;
+        return scde_b200_batch_boot_indices(seeds[set], L, bp.off.data(), bp.pool.data(), bcomp[b].data(), a->n_boot,
+                                            p.bdraws.data() + p.bdraw_off[b] + (int64_t)set * a->n_boot * p.bslot_D[b]);
+    }));
     p.pair_bslot.resize(p.pair_slot.size());
     for (size_t i = 0; i < p.pair_slot.size(); ++i) p.pair_bslot[i] = bslot_of_slot[p.pair_slot[i]];
     if (a->batch_models) {

@@ -294,6 +294,8 @@ struct TiledParams {
     int64_t ld_lst;
     const double *W;  // this pass: rows [n_w_rows][108], columns [0, 104) real
     const double *Z;  // this pass: [104][416] initial value of T (zero-base form) or NULL
+    const int32_t *gene_set;  // draw set of every gene (NULL: one set): W rows and Z of set s start s * set_w_rows rows and
+    int64_t set_w_rows, set_z;  // s * set_z doubles after W and Z
     double *T;        // [n_pos][104][416]: T[b, k] of the gene at position `pos` of `order` (this launch's chunk)
     int n_pos;        // genes in this launch: positions [0, n_pos) of `order`
     int debug;  // timing experiments only (SCDE_B200_DEBUG_CONTRACT): 1 = no DMMA, 2 = no table-row copies
@@ -374,8 +376,10 @@ __device__ __forceinline__ void run_mma(const TiledParams &p, MmaSmem &sm, int w
     };
     auto fetch_entries = [&](int i, int cb) -> int32_t {
         if (lane < 2 * T_S && i < n_my) {
-            const int64_t o = gene_of(item_of(i)) * p.ld_lst + (int64_t)cb * T_S + (lane & (T_S - 1));
-            return lane < T_S ? p.lst_row[o] : p.lst_cell[o];
+            const int64_t gene = gene_of(item_of(i));
+            const int64_t o = gene * p.ld_lst + (int64_t)cb * T_S + (lane & (T_S - 1));
+            if (lane < T_S) return p.lst_row[o];
+            return p.lst_cell[o] + (p.gene_set ? (int32_t)(p.gene_set[gene] * p.set_w_rows) : 0);
         }
         return 0;
     };
@@ -419,12 +423,14 @@ __device__ __forceinline__ void run_mma(const TiledParams &p, MmaSmem &sm, int w
         const int spg = (p.lst_len[gene_of(item)] + T_S - 1) / T_S;
         double acc[2][M_NT][2];
         double ex[M_NEX][2];
-        if (p.Z) {  // zero-base form: T starts from the per-randomization sum of the zero-count rows
+        const double *Zg = p.Z;
+        if (Zg && p.gene_set) Zg += p.gene_set[gene_of(item)] * p.set_z;
+        if (Zg) {  // zero-base form: T starts from the per-randomization sum of the zero-count rows
 #pragma unroll
             for (int nt = 0; nt < M_NT; ++nt)
 #pragma unroll
                 for (int i = 0; i < 2; ++i) {
-                    const double *z = p.Z + (int64_t)(nt * 8 + 2 * t + i) * KP_TILED + kbase + g;
+                    const double *z = Zg + (int64_t)(nt * 8 + 2 * t + i) * KP_TILED + kbase + g;
                     acc[0][nt][i] = z[(m0 + 0) * 8];
                     acc[1][nt][i] = z[(m0 + 1) * 8];
                 }
@@ -432,7 +438,7 @@ __device__ __forceinline__ void run_mma(const TiledParams &p, MmaSmem &sm, int w
             for (int j = 0; j < M_NEX; ++j)
 #pragma unroll
                 for (int i = 0; i < 2; ++i)
-                    ex[j][i] = p.Z[(int64_t)((nx0 + (j < nex ? j : 0)) * 8 + 2 * t + i) * KP_TILED + kbase + mx * 8 + g];
+                    ex[j][i] = Zg[(int64_t)((nx0 + (j < nex ? j : 0)) * 8 + 2 * t + i) * KP_TILED + kbase + mx * 8 + g];
         } else {
 #pragma unroll
             for (int nt = 0; nt < M_NT; ++nt) {
@@ -589,6 +595,8 @@ struct GenericParams {
     const double *W;  // pass-major [pass][n_w_rows][108]
     int64_t n_w_rows;
     const double *Z;  // [passes*104][ld_table] or NULL
+    const int32_t *gene_set;  // as in TiledParams
+    int64_t set_w_rows, set_z;
     int n_boot;
     double scale;
     int K;
@@ -599,14 +607,16 @@ struct GenericParams {
 __device__ __forceinline__ void generic_accumulate(const GenericParams &p, int64_t g, int b0, int k0,
                                                    double (&acc)[G_KPT][G_BC]) {
     const int pass = b0 / WP_TILED, bb = b0 % WP_TILED;
+    const int64_t set = p.gene_set ? p.gene_set[g] : 0;
+    const double *Z = p.Z ? p.Z + set * p.set_z : nullptr;
 #pragma unroll
     for (int i = 0; i < G_KPT; ++i)
 #pragma unroll
         for (int j = 0; j < G_BC; ++j) {
             const int k = k0 + i * G_THREADS;
-            acc[i][j] = (p.Z && k < p.K) ? p.Z[((int64_t)pass * WP_TILED + bb + j) * p.ld_table + k] : 0.0;
+            acc[i][j] = (Z && k < p.K) ? Z[((int64_t)pass * WP_TILED + bb + j) * p.ld_table + k] : 0.0;
         }
-    const double *Wc = p.W + ((int64_t)pass * p.n_w_rows) * WS_TILED + bb;
+    const double *Wc = p.W + (set * p.set_w_rows + (int64_t)pass * p.n_w_rows) * WS_TILED + bb;
     const int len = p.lst_len[g];
     for (int e = 0; e < len; ++e) {
         const int64_t row = p.lst_row[g * p.ld_lst + e];
@@ -932,6 +942,9 @@ cudaError_t launch_contract_tiled(const ContractArgs &a, int n_sm, double *t_scr
             p.ld_lst = a.lists.ld;
             p.W = a.W + (size_t)ps * a.n_w_rows * WS_TILED;
             p.Z = a.Z ? a.Z + (size_t)ps * WP_TILED * KP_TILED : nullptr;
+            p.gene_set = a.gene_set;
+            p.set_w_rows = a.set_w_rows;
+            p.set_z = a.set_z;
             p.T = t_scratch;
             p.n_pos = n_pos;
             p.debug = a.debug;
@@ -976,6 +989,9 @@ cudaError_t launch_contract_generic(const ContractArgs &a, cudaStream_t st, int 
     p.W = a.W;
     p.n_w_rows = a.n_w_rows;
     p.Z = a.Z;
+    p.gene_set = a.gene_set;
+    p.set_w_rows = a.set_w_rows;
+    p.set_z = a.set_z;
     p.n_boot = a.n_boot;
     p.scale = a.scale;
     p.K = a.K;

@@ -130,6 +130,10 @@ struct ContractArgs {
     int n_w_rows;
     int n_boot;       // columns of W that are real
     const double *Z;  // [ceil(n_boot/104)*104][ld_table] initial value of T, or NULL (dense lists)
+    // Draw sets: gene_set[gene] (NULL: one set) selects the W and Z of the gene's set, which start gene_set[gene] *
+    // set_w_rows rows of W ([set][pass][n_w_rows][108]) and gene_set[gene] * set_z doubles of Z after the first set's
+    const int32_t *gene_set;
+    int64_t set_w_rows, set_z;
     double scale;     // jp += softmax / scale   (n_boot for the live path, 1 for the legacy / no-bootstrap forms)
     int n_genes, K;
     double *jp;  // [n_genes][ld_jp], must be zeroed by the caller
@@ -192,6 +196,10 @@ struct ContractI8Args {
     int n_w_rows;
     int n_boot;
     const double *Z;   // [ceil(n_boot/104)*104][416] or NULL
+    // Draw sets: gene_set[gene] (NULL: one set) selects the W8 and Z of the gene's set, gene_set[gene] * set_w8 bytes and
+    // gene_set[gene] * set_z doubles after the first set's (W8 [set][pass][n_w_rows][128]; the twin's W8 likewise)
+    const int32_t *gene_set;
+    int64_t set_w8, set_z;
     double scale;
     double sentinel;   // the "log 0" value of the FP64 table
     int n_genes, K;

@@ -81,6 +81,8 @@ struct I8Params {
     const int32_t *lst_row, *lst_cell, *lst_len, *order;
     int64_t ld_lst;
     const int8_t *W8;    // this pass: [n_w_rows][128]
+    const int32_t *gene_set;  // draw set of every gene (NULL: one set): its W rows start gene_set[gene] * set_w8 bytes
+    int64_t set_w8;           // after W8 (and W8b)
     long long *T;        // [n_pos][104][416]: 2^29 * T[boot, grid] as exact integers (without Z, without sentinels)
     int n_boot;          // real boots of this pass: rows beyond are not stored
     int n_pos;           // genes in this launch: positions [0, n_pos) of `order`
@@ -179,22 +181,24 @@ __device__ __forceinline__ void run_producer(const I8Params &p, I8Smem &sm, uint
     int slot_b = 0;        // ring slot of the first stage of the current item
     uint32_t fill_b = 0;   // how often that slot has been filled before
     int item = blockIdx.x;
-    int64_t gene_n = 0;
+    int64_t gene_n = 0, wset_n = 0;  // wset: byte offset of the gene's draw set in W8
     int len_n = 0;
     if (item < n_items) {
         gene_n = item_gene(p, item);
         len_n = p.lst_len[gene_n];
+        if (p.gene_set) wset_n = p.gene_set[gene_n] * p.set_w8;
     }
     for (; item < n_items; item += gridDim.x) {
         const Item it = decode_item(p, item);
-        const int64_t gene = gene_n;
+        const int64_t gene = gene_n, wset = wset_n;
         const int nst = (len_n + Q_ES - 1) / Q_ES;
         if (item + (int)gridDim.x < n_items) {
             gene_n = item_gene(p, item + gridDim.x);
             len_n = p.lst_len[gene_n];
+            if (p.gene_set) wset_n = p.gene_set[gene_n] * p.set_w8;
         }
         const int8_t *qbase = p.qtable + (int64_t)it.piece * Q_PIECE + l7 * 16;
-        const int8_t *wbase = ((p.twin && (item & 1)) ? p.W8b : p.W8) + l7 * 16;
+        const int8_t *wbase = ((p.twin && (item & 1)) ? p.W8b : p.W8) + l7 * 16 + wset;
         const int32_t *lrow = p.lst_row + gene * p.ld_lst + kg * 8 + l3;
         const int32_t *lcell = p.lst_cell + gene * p.ld_lst + kg * 8 + l3;
         int32_t r0a = 0, r1a = 0, c0a = 0, c1a = 0, r0b = 0, r1b = 0, c0b = 0, c1b = 0;
@@ -451,12 +455,14 @@ __global__ void __launch_bounds__(q_threads(Q_PGROUPS), 1) contract_i8_kernel(co
 __global__ void __launch_bounds__(256) sentinel_range_kernel(const int32_t *__restrict__ lst_row, const int32_t *__restrict__ lst_cell,
                                                              const int32_t *__restrict__ lst_len, const int32_t *__restrict__ order,
                                                              int64_t ld_lst, const uint32_t *__restrict__ row_range,
-                                                             const int8_t *__restrict__ W8, int n_pos, int K, int n_boot,
+                                                             const int8_t *__restrict__ W8, const int32_t *__restrict__ gene_set,
+                                                             int64_t set_w8, int n_pos, int K, int n_boot,
                                                              uint32_t *__restrict__ SR, int32_t *__restrict__ flag) {
     const int pos = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (pos >= n_pos) return;
     const int lane = threadIdx.x & 31;
     const int64_t gene = order ? order[pos] : pos;
+    if (gene_set) W8 += gene_set[gene] * set_w8;  // the W rows of the gene's draw set
     const int len = lst_len[gene];
     const int32_t *lr = lst_row + gene * ld_lst, *lc = lst_cell + gene * ld_lst;
     const uint32_t full = (uint32_t)(K - 1) << 16;
@@ -547,19 +553,25 @@ static_assert(SP_GROUPS * SP_ROWS == WP_TILED && SP_ROWS * 32 == KP_TILED, "13 w
 // boot's row is already in flight), soft-max pieces by shuffles (exp_nonpos, skipped warp-wide where a 32-point stretch
 // lies > 746 nats below the row maximum: a joint posterior is sharply peaked), and the normalised row is added to 13
 // accumulators per lane in ascending boot order.
+// SETS (several draw sets, DESIGN.md "Draw sets"): each gene reads the Z rows of its own set, gene_set[gene] * set_z doubles
+// after Z, from global memory (L2) instead of shared memory -- the same values in the same order, so the same result.
 constexpr int SW_WARPS = 8;
+template <bool SETS>
 __global__ void __launch_bounds__(SW_WARPS * 32, 2)
 softmax_i8_warp_kernel(const long long *__restrict__ T, const double *__restrict__ Z, const uint32_t *__restrict__ SR, int K,
-                       int n_boot_pass, double scale, double *__restrict__ part, int n_pos) {
+                       int n_boot_pass, double scale, double *__restrict__ part, int n_pos, const int32_t *__restrict__ order,
+                       const int32_t *__restrict__ gene_set, int64_t set_z) {
     constexpr int NJ = KP_TILED / 32;
-    extern __shared__ double s_z[];  // [SP_ROWS][KP_TILED]
+    extern __shared__ double s_z[];  // [SP_ROWS][KP_TILED] (one set only)
     const int group = blockIdx.x % SP_GROUPS, batch = blockIdx.x / SP_GROUPS, n_batch = gridDim.x / SP_GROUPS;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int b0 = group * SP_ROWS;
     const int nb = min(SP_ROWS, n_boot_pass - b0);  // boots of this group (<= 0: none)
-    for (int i = threadIdx.x; i < SP_ROWS * KP_TILED; i += SW_WARPS * 32)
-        s_z[i] = (Z && i / KP_TILED < nb) ? Z[(int64_t)b0 * KP_TILED + i] : 0.0;
-    __syncthreads();
+    if (!SETS) {
+        for (int i = threadIdx.x; i < SP_ROWS * KP_TILED; i += SW_WARPS * 32)
+            s_z[i] = (Z && i / KP_TILED < nb) ? Z[(int64_t)b0 * KP_TILED + i] : 0.0;
+        __syncthreads();
+    }
     const double q = 1.0 / (double)(1ll << Q_FRAC);
     for (int pos = batch * SW_WARPS + warp; pos < n_pos; pos += n_batch * SW_WARPS) {
         double acc[NJ];
@@ -568,6 +580,8 @@ softmax_i8_warp_kernel(const long long *__restrict__ T, const double *__restrict
         const long long *rows = T + ((int64_t)pos * WP_TILED + b0) * KP_TILED + lane;
         // the group's 13 range words, one per lane
         const uint32_t sr_l = (SR && lane < SP_ROWS) ? SR[(int64_t)pos * Q_WB + b0 + lane] : 0xFFFF0000u;
+        const double *zg = s_z;
+        if (SETS) zg = Z + gene_set[order ? order[pos] : pos] * set_z + (int64_t)b0 * KP_TILED;
         long long nxt[NJ];
         if (nb > 0) {
 #pragma unroll
@@ -584,7 +598,7 @@ softmax_i8_warp_kernel(const long long *__restrict__ T, const double *__restrict
             }
             const uint32_t sr = __shfl_sync(0xffffffffu, sr_l, bi);
             const int klo = (int)(sr & 0xFFFFu), span = min((int)(sr >> 16), K - 1) - klo;  // admissible: klo .. klo + span
-            const double *zr = s_z + bi * KP_TILED + lane;
+            const double *zr = zg + bi * KP_TILED + lane;
             double v[NJ], m = -INFINITY;
 #pragma unroll
             for (int j = 0; j < NJ; ++j) {
@@ -754,6 +768,8 @@ static I8Params make_params(const ContractI8Args &a, int g0, int n_pos, int pass
     p.order = a.lists.order ? a.lists.order + g0 : nullptr;
     p.ld_lst = a.lists.ld;
     p.W8 = a.W8 + (size_t)pass * a.n_w_rows * Q_WB;
+    p.gene_set = a.gene_set;
+    p.set_w8 = a.set_w8;
     p.T = reinterpret_cast<long long *>(t_scratch);
     p.n_boot = (a.n_boot - pass * WP_TILED) < WP_TILED ? (a.n_boot - pass * WP_TILED) : WP_TILED;
     p.n_pos = n_pos;
@@ -775,7 +791,8 @@ cudaError_t launch_sentinel_ranges(const ContractI8Args &a, int g0, int n_pos, i
     const I8Params p = make_params(a, g0, n_pos, pass, nullptr);
     const int nb = (a.n_boot - pass * WP_TILED) < WP_TILED ? (a.n_boot - pass * WP_TILED) : WP_TILED;
     sentinel_range_kernel<<<(unsigned)((n_pos + 7) / 8), 256, 0, st>>>(p.lst_row, p.lst_cell, p.lst_len, p.order, p.ld_lst,
-                                                                       a.row_range, p.W8, n_pos, a.K, nb, sr_scratch, a.err);
+                                                                       a.row_range, p.W8, a.gene_set, a.set_w8, n_pos, a.K,
+                                                                       nb, sr_scratch, a.err);
     return cudaGetLastError();
 }
 
@@ -817,15 +834,17 @@ cudaError_t launch_softmax_i8(const ContractI8Args &a, int g0, int n_pos, int pa
     if (a.row_range && !sr) return cudaErrorInvalidValue;
     const int nb = (a.n_boot - pass * WP_TILED) < WP_TILED ? (a.n_boot - pass * WP_TILED) : WP_TILED;
     const double *Z = a.Z ? a.Z + (size_t)pass * WP_TILED * KP_TILED : nullptr;
-    const size_t smem = sizeof(double) * SP_ROWS * KP_TILED;
-    cudaError_t e = cudaFuncSetAttribute(softmax_i8_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    const bool sets = a.gene_set && Z;
+    const size_t smem = sets ? 0 : sizeof(double) * SP_ROWS * KP_TILED;
+    auto kernel = sets ? softmax_i8_warp_kernel<true> : softmax_i8_warp_kernel<false>;
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     int wb = n_sm * 2 / SP_GROUPS;  // two CTAs of eight warps per SM
     if (wb * SW_WARPS > n_pos) wb = (n_pos + SW_WARPS - 1) / SW_WARPS;
     if (wb < 1) wb = 1;
-    softmax_i8_warp_kernel<<<wb * SP_GROUPS, SW_WARPS * 32, smem, st>>>(reinterpret_cast<const long long *>(t_scratch), Z,
-                                                                        a.row_range ? sr : nullptr, a.K, nb, a.scale,
-                                                                        part_scratch, n_pos);
+    kernel<<<wb * SP_GROUPS, SW_WARPS * 32, smem, st>>>(reinterpret_cast<const long long *>(t_scratch), Z,
+                                                        a.row_range ? sr : nullptr, a.K, nb, a.scale, part_scratch, n_pos,
+                                                        a.lists.order ? a.lists.order + g0 : nullptr, a.gene_set, a.set_z);
     e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     const int64_t n = (int64_t)n_pos * KP_TILED;
