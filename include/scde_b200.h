@@ -117,7 +117,9 @@ typedef struct {
     int32_t twin_batch_joints;  /* 1 (default): two contractions over the same cells and rows share the launches of the tcgen05
                                    kernel (paired items on neighbouring SMs): the two composition-sampled joints of a
                                    batch-corrected call, and the two passes of more than 104 randomizations */
-    int32_t reserved[5];
+    int32_t prune_pieces;       /* 1 (default): the tcgen05 contraction skips the (gene, piece) items whose grid points bounds
+                                   computed before it prove invisible to the soft-max (DESIGN.md 4.3); results are unchanged */
+    int32_t reserved[4];
 } scde_b200_options;
 SCDE_B200_API int scde_b200_get_options(const scde_b200_ctx *ctx, scde_b200_options *opt);
 SCDE_B200_API int scde_b200_set_options(scde_b200_ctx *ctx, const scde_b200_options *opt);
@@ -264,6 +266,7 @@ enum {
     SCDE_B200_T_RATIO,       /* sliding product + summary (all passes) */
     SCDE_B200_T_OTHER,       /* W build, entry lists, zero-count base sums, memsets */
     SCDE_B200_T_SOFTMAX,     /* soft-max over the grid + average over boots after the tcgen05 contraction kernel */
+    SCDE_B200_T_BOUND,       /* pruning before the tcgen05 contraction: bound pass, live-item decision and list */
     SCDE_B200_T_TOTAL,
     SCDE_B200_T_COUNT
 };
@@ -272,6 +275,12 @@ typedef struct {
     int32_t launches[SCDE_B200_T_COUNT];
     int64_t table_rows;      /* rows in the log-posterior table */
     int64_t contract_cells;  /* list entries (gene x cell pairs) the contraction visited, summed over all joints */
+    int64_t prune_items;     /* (gene, piece) items of the pruned tcgen05 launches, summed over joints and passes (a twin
+                                launch counts its pairs once) */
+    int64_t prune_live;      /* ... of which were contracted */
+    int64_t prune_work;      /* the same items weighted by their gene's list length: (visited pair, piece) units, i.e. the
+                                gather the launches would have done unpruned */
+    int64_t prune_live_work; /* ... of which were gathered */
 } scde_b200_stats;
 
 /* One-shot: host buffers in, host buffers out (uploads, runs, downloads).  The count matrix goes up in cell chunks that are
@@ -420,6 +429,22 @@ SCDE_B200_API int scde_b200_probe_contract_i8(scde_b200_ctx *ctx, const int8_t *
                                 const uint32_t *row_range, const int8_t *w8, int32_t n_w_rows, const int32_t *lst_row,
                                 const int32_t *lst_cell, const int32_t *lst_len, int32_t n_genes, int32_t ld_lst,
                                 double *t_out, int32_t *flags_out);
+/* scde_b200_probe_table plus qbound_out[n_rows][128]: the bound row of every fixed-point row (DESIGN.md 4.3, "Pruned
+ * pieces"; layout in csrc/common.cuh), as the differential-expression call writes it. */
+SCDE_B200_API int scde_b200_probe_table_bounds(scde_b200_ctx *ctx, const double *models, int32_t n_cells, const int32_t *ucl_flat,
+                         const int32_t *ucl_offsets, const double *magnitudes, int32_t n_grid, int32_t local_theta,
+                         int32_t square_logit_conc, int32_t n_cells_for_clamp, int8_t *q_out, uint32_t *row_range_out,
+                         int32_t *zero_row_out, int32_t *based_out, double *zero_rows_out, int8_t *qbound_out);
+/* scde_b200_probe_contract_i8 (t_out is the UNPRUNED T, without z) plus, when qbound (the bound rows of qtable) is given,
+ * the pruning decision for the same launch: z[104][416] (or NULL: 0) is the zero-count base the soft-max would add;
+ * lb_out[n_genes][104] the lower bound on every boot's row maximum, ub_out[n_genes][104][4] the upper bound on every
+ * piece's admissible T (-inf: none), live_out[n_genes] bit p = piece p is contracted.  exp_out (may be NULL): exp_nonpos at
+ * -745, -746 and -747 as the soft-max evaluates it on the device. */
+SCDE_B200_API int scde_b200_probe_prune_i8(scde_b200_ctx *ctx, const int8_t *qtable, int32_t n_rows, int32_t n_grid,
+                             const uint32_t *row_range, const int8_t *qbound, const double *z, const int8_t *w8,
+                             int32_t n_w_rows, const int32_t *lst_row, const int32_t *lst_cell, const int32_t *lst_len,
+                             int32_t n_genes, int32_t ld_lst, double *t_out, double *lb_out, double *ub_out,
+                             uint8_t *live_out, double *exp_out, int32_t *flags_out);
 
 #ifdef __cplusplus
 }

@@ -13,8 +13,8 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("SCDE_B200_LIB") or os.path.join(_HERE, "libscde_b200.so")
 
-T_DEDUP, T_LPTABLE, T_CONTRACT, T_RATIO, T_OTHER, T_SOFTMAX, T_TOTAL, T_COUNT = range(8)
-STAGE_NAMES = ["dedup", "lp_table", "contract", "ratio", "other", "softmax", "total"]
+T_DEDUP, T_LPTABLE, T_CONTRACT, T_RATIO, T_OTHER, T_SOFTMAX, T_BOUND, T_TOTAL, T_COUNT = range(9)
+STAGE_NAMES = ["dedup", "lp_table", "contract", "ratio", "other", "softmax", "bound", "total"]
 
 i32p = C.POINTER(C.c_int32)
 f64p = C.POINTER(C.c_double)
@@ -86,12 +86,16 @@ class ContrastOut(C.Structure):
 
 class Stats(C.Structure):
     _fields_ = [("ms", C.c_float * T_COUNT), ("launches", C.c_int32 * T_COUNT),
-                ("table_rows", C.c_int64), ("contract_cells", C.c_int64)]
+                ("table_rows", C.c_int64), ("contract_cells", C.c_int64),
+                ("prune_items", C.c_int64), ("prune_live", C.c_int64),
+                ("prune_work", C.c_int64), ("prune_live_work", C.c_int64)]
 
     def as_dict(self):
         return {"ms": {STAGE_NAMES[i]: float(self.ms[i]) for i in range(T_COUNT - 1)},
                 "launches": {STAGE_NAMES[i]: int(self.launches[i]) for i in range(T_COUNT - 1)},
-                "table_rows": int(self.table_rows), "contract_cells": int(self.contract_cells)}
+                "table_rows": int(self.table_rows), "contract_cells": int(self.contract_cells),
+                "prune_items": int(self.prune_items), "prune_live": int(self.prune_live),
+                "prune_work": int(self.prune_work), "prune_live_work": int(self.prune_live_work)}
 
 
 class Options(C.Structure):
@@ -99,7 +103,7 @@ class Options(C.Structure):
     _fields_ = [(n, C.c_int32) for n in (
         "contract_kernel", "zero_base", "fused_fixed_point", "lp_rows_kernel", "count_chunks", "split_front",
         "uniform_chunks", "pipeline_front", "item_order", "hot_rank", "cold_evict_first", "trace", "epilogue_timing",
-        "debug_contract", "ring_stages", "twin_batch_joints")] + [("reserved", C.c_int32 * 5)]
+        "debug_contract", "ring_stages", "twin_batch_joints", "prune_pieces")] + [("reserved", C.c_int32 * 4)]
 
 
 # every symbol include/scde_b200.h declares
@@ -112,6 +116,7 @@ EXPORTED = [
     "scde_b200_bh_cz", "scde_b200_expression_difference", "scde_b200_diff_upload", "scde_b200_diff_run",
     "scde_b200_diff_download", "scde_b200_diff_free", "scde_b200_expression_magnitude", "scde_b200_cell_table",
     "scde_b200_measure_fp64_peak", "scde_b200_set_contract_kernel", "scde_b200_probe_contract_i8", "scde_b200_probe_table",
+    "scde_b200_probe_table_bounds", "scde_b200_probe_prune_i8",
     "scde_b200_failure_probability", "scde_b200_expression_prior", "scde_b200_dataset_create",
     "scde_b200_dataset_contrasts", "scde_b200_dataset_free",
 ]
@@ -155,6 +160,9 @@ def lib():
         L.scde_b200_n_devices.argtypes = [C.c_void_p]
         L.scde_b200_probe_table.argtypes = [C.c_void_p, f64p, C.c_int32, i32p, i32p, f64p, C.c_int32, C.c_int32, C.c_int32,
                                             C.c_int32, C.c_void_p, C.c_void_p, i32p, i32p, f64p]
+        L.scde_b200_probe_table_bounds.argtypes = L.scde_b200_probe_table.argtypes + [C.c_void_p]
+        L.scde_b200_probe_prune_i8.argtypes = [C.c_void_p] + [C.c_void_p] + [C.c_int32] * 2 + [C.c_void_p] * 4 + [C.c_int32] + \
+            [C.c_void_p] * 3 + [C.c_int32] * 2 + [C.c_void_p] * 6
         L.scde_b200_get_options.argtypes = [C.c_void_p, C.POINTER(Options)]
         L.scde_b200_set_options.argtypes = [C.c_void_p, C.POINTER(Options)]
         _lib = L

@@ -137,6 +137,7 @@ static scde_b200_options default_options() {
     o.hot_rank = -1;
     o.cold_evict_first = 1;
     o.twin_batch_joints = 1;
+    o.prune_pieces = 1;
     return o;
 }
 
@@ -167,9 +168,12 @@ struct LpTable {
     DBuf<double> table, mu, lcfp, lcfpr, theta, maxcfp, cfp, l1, l2, rowc, scfp;
     DBuf<int8_t> q;      // fixed-point planes of the table (contract_i8.cu), [n_rows][q_row_bytes(K)]
     DBuf<uint32_t> qrange;  // [n_rows] non-sentinel range of every row (klo | khi << 16)
+    DBuf<int8_t> qb;        // [n_rows][Q_BW] bound rows of the fixed-point table (pruned contraction)
     DBuf<uint32_t> dedup_bits;  // per-cell bitmaps between the two dedup passes
     DBuf<unsigned long long> work_counter;  // chunk counter of the fixed-point row kernel
     bool want_q = false, has_q = false;
+    bool want_bounds = false;  // bound rows whatever the size (scde_b200_probe_table_bounds)
+    bool has_bounds = false;   // t.qb holds the bound rows of the fixed-point table
     bool f64_rows = true;  // false: the FP64 rows of non-zero counts were not stored (planes only)
     bool want_modes = true;  // row_mode (argmax of every row) is needed: only for return.individual.posterior.modes
     bool fast_theta = false;  // every corr.theta finite and > 0, no local-theta fit: constant-theta fast path
@@ -197,6 +201,11 @@ struct LpTable {
     } while (0)
 
 // What fill_table decides once per table and the row-level launches need: which kernels, which outputs.
+// Pruning (DESIGN.md 4.3) pays where a joint has at least this many cells: measured on one B200 (1000 W), config 3 (1000
+// cells per joint) was 3.0 ms per step slower with it (bound pass and bound rows cost more than the 27 % of the gather they
+// removed), config 4 (5000) 7.7 ms faster.  The bound rows are only written for tables of at least as many cells.
+constexpr int PRUNE_MIN_CELLS = 2500;
+
 struct TablePlan {
     bool fast = false;     // constant-theta fast row kernel
     bool q_any = false;    // the table also exists in fixed point (tcgen05 contraction)
@@ -206,6 +215,8 @@ struct TablePlan {
     int32_t *rmode = nullptr;
     int8_t *qf = nullptr;
     uint32_t *qr = nullptr;
+    int8_t *qb = nullptr;
+    bool bounds = false;   // the table also gets its bound rows
 };
 
 TablePlan plan_table(const scde_b200_ctx *ctx, const LpTable &t, int local_theta) {
@@ -213,6 +224,7 @@ TablePlan plan_table(const scde_b200_ctx *ctx, const LpTable &t, int local_theta
     pl.fast = t.fast_theta && !local_theta && t.K <= KP_TILED;
     pl.q_any = t.want_q && t.zero_base && t.ld == KP_TILED && t.K <= Q_MAX_K;
     pl.q_fused = pl.q_any && pl.fast && ctx->opt.fused_fixed_point;
+    pl.bounds = pl.q_any && (t.want_bounds || (ctx->opt.prune_pieces && t.n_cells >= PRUNE_MIN_CELLS));
     return pl;
 }
 
@@ -256,12 +268,15 @@ int reserve_rows(LpTable &t, TablePlan &pl, size_t rows) {
     if (pl.q_any) {
         SCDE_CUDA(t.q.ensure(rows * q_row_bytes(t.K)));
         SCDE_CUDA(t.qrange.ensure(rows));
+        if (pl.bounds) SCDE_CUDA(t.qb.ensure(rows * Q_BW));
         SCDE_CUDA(t.work_counter.ensure(1));
     }
     pl.rowc = pl.fast ? (void *)t.rowc.p : nullptr;
     pl.rmode = t.want_modes ? t.row_mode.p : nullptr;
     pl.qf = pl.q_fused ? t.q.p : nullptr;
     pl.qr = pl.q_fused ? t.qrange.p : nullptr;
+    pl.qb = pl.q_fused && pl.bounds ? t.qb.p : nullptr;
+    t.has_bounds = pl.bounds;
     return SCDE_B200_OK;
 }
 
@@ -282,13 +297,13 @@ int launch_table_rows(scde_b200_ctx *ctx, const LpTable &t, const TablePlan &pl,
         SCDE_CUDA(launch_zero_rows(t.row_off.p + cr.c0, t.row_x.p, n, t.zero_row.p + cr.c0, cr.row_cap, st));
         SCDE_CUDA(launch_lp_rows(models_dev, ld_models, cr, t.row_off.p, t.row_cell.p, t.row_x.p, pl.prep, t.K, local_theta,
                                  t.sentinel, t.table.p, t.ld, pl.rmode, 1, t.zero_row.p, nullptr, pl.rowc, t.row_snap.p, 1, pl.qf, pl.qr,
-                                 st, 0, nullptr, t.zero_compact));
+                                 st, 0, nullptr, t.zero_compact, pl.qb));
         SCDE_CUDA(launch_based_flags(t.table.p, t.ld, t.K, t.sentinel, t.zero_row.p + cr.c0, n, t.based.p + cr.c0, st,
                                      t.zero_compact ? cr.c0 : -1));
         SCDE_CUDA(launch_lp_rows(models_dev, ld_models, cr, t.row_off.p, t.row_cell.p, t.row_x.p, pl.prep, t.K, local_theta,
                                  t.sentinel, t.table.p, t.ld, pl.rmode, 2, t.zero_row.p, t.based.p, pl.rowc, t.row_snap.p,
                                  pl.q_fused ? 0 : 1, pl.qf, pl.qr, st, ctx->opt.lp_rows_kernel == 1, t.work_counter.p,
-                                 t.zero_compact));
+                                 t.zero_compact, pl.qb));
         *nl += 4;
     } else {
         SCDE_CUDA(launch_lp_rows(models_dev, ld_models, cr, t.row_off.p, t.row_cell.p, t.row_x.p, pl.prep, t.K, local_theta,
@@ -314,7 +329,7 @@ int fill_table(scde_b200_ctx *ctx, LpTable &t, const double *models_dev, int ld_
     t.has_q = pl.q_any;
     t.f64_rows = !(pl.q_fused && t.zero_base);
     if (pl.q_any && !pl.q_fused) {
-        SCDE_CUDA(launch_quantize_rows(t.table.p, t.ld, t.K, t.n_rows, t.q.p, t.qrange.p, st));
+        SCDE_CUDA(launch_quantize_rows(t.table.p, t.ld, t.K, t.n_rows, t.q.p, t.qrange.p, pl.bounds ? t.qb.p : nullptr, st));
         ++nl;
     }
     if (tm) tm->end(SCDE_B200_T_LPTABLE, e0, st, nl);
@@ -389,7 +404,12 @@ struct JointScratch {
     DBuf<uint32_t> SR;  // sentinel range of every (gene, boot) of one launch of the tcgen05 kernel
     DBuf<uint32_t> SR2;
     DBuf<int32_t> lst_row, lst_cell, lst_len, order;
-    DBuf<unsigned long long> total;  // running sum of list lengths over the joints of one run
+    DBuf<unsigned long long> total;  // running sums over the joints of one run: list lengths, then launch_prune_items' four
+    // pruning (launch_prune_items): Z extrema of the joint, bound sums of one launch (S2: the paired pass), live pieces and
+    // items of one launch, and the live count
+    DBuf<double> zb;
+    DBuf<int32_t> S, S2, items, n_live;
+    DBuf<uint8_t> live;
 };
 
 // The big allocations of scde.expression.difference (counts shard, index matrix, lp table, joint posteriors, ratio
@@ -424,9 +444,11 @@ struct TwinJoint {
 
 // The tcgen05 contraction of a joint whose operands run_joint has prepared, and of its twin (NULL: none) in the same
 // launches.  The launches raise bits in *status (read_status).
+// prune (DESIGN.md 4.3): before each launch a bound pass and a decision find the (gene, piece) items the soft-max cannot
+// see; the contraction and the soft-max then skip them.  prune_stats (or NULL): launch_prune_items' four counters.
 int contract_joint_i8(scde_b200_ctx *ctx, const LpTable &t, const GeneLists &lists, JointScratch &scr, int n_w_rows,
                       int n_boot, const DrawSets &sets, double scale, double *jp_dev, int ld_jp, int hot_rank,
-                      int32_t *status, const TwinJoint *twin, StageTimer *tm) {
+                      int32_t *status, const TwinJoint *twin, StageTimer *tm, bool prune, unsigned long long *prune_stats) {
     cudaStream_t st = ctx->stream;
     const int passes = (n_boot + WP_TILED - 1) / WP_TILED;
     ContractI8Args q{};
@@ -481,6 +503,25 @@ int contract_joint_i8(scde_b200_ctx *ctx, const LpTable &t, const GeneLists &lis
         SCDE_CUDA(scr.T2.ensure(contract_tiled_scratch_doubles(t.n_genes)));
         SCDE_CUDA(scr.SR2.ensure(contract_i8_range_words(t.n_genes < max_genes ? t.n_genes : max_genes)));
     }
+    if (prune) {
+        const int mp = t.n_genes < max_genes ? t.n_genes : max_genes;
+        q.qbound = t.qb.p;
+        SCDE_CUDA(scr.zb.ensure(prune_zb_doubles(sets.n, n_boot)));
+        SCDE_CUDA(scr.S.ensure(prune_bound_ints(mp)));
+        if (pass_pairs) SCDE_CUDA(scr.S2.ensure(prune_bound_ints(mp)));
+        SCDE_CUDA(scr.live.ensure((size_t)mp));
+        SCDE_CUDA(scr.items.ensure((size_t)mp * q_pieces(t.K)));
+        SCDE_CUDA(scr.n_live.ensure(1));
+        const int e0 = tm ? tm->begin(st) : -1;
+        SCDE_CUDA(launch_z_bounds(q, sets.n, scr.zb.p, st));
+        if (twin) {
+            JointScratch &s2 = *twin->scr;
+            SCDE_CUDA(s2.zb.ensure(prune_zb_doubles(sets.n, n_boot)));
+            SCDE_CUDA(s2.S.ensure(prune_bound_ints(mp)));
+            SCDE_CUDA(launch_z_bounds(q2, sets.n, s2.zb.p, st));
+        }
+        if (tm) tm->end(SCDE_B200_T_BOUND, e0, st, twin ? 2 : 1);
+    }
     for (int g0 = 0; g0 < t.n_genes; g0 += max_genes) {
         const int n_pos = (t.n_genes - g0) < max_genes ? (t.n_genes - g0) : max_genes;
         for (int ps = 0; ps < passes; ++ps) {
@@ -490,24 +531,40 @@ int contract_joint_i8(scde_b200_ctx *ctx, const LpTable &t, const GeneLists &lis
             if (twin) SCDE_CUDA(launch_sentinel_ranges(q2, g0, n_pos, ps, twin->scr->SR.p, st));
             if (pair) SCDE_CUDA(launch_sentinel_ranges(q, g0, n_pos, ps + 1, scr.SR2.p, st));
             if (tm) tm->end(SCDE_B200_T_OTHER, e0, st, (twin || pair) ? 2 : 1);
-            e0 = tm ? tm->begin(st) : -1;
             if (pair) {  // make_params adds the pass offset to both W pointers: the twin is the next pass
                 q.W8_twin = q.W8 + (size_t)n_w_rows * Q_WB;
                 q.t_twin = scr.T2.p;
             }
+            if (prune) {
+                e0 = tm ? tm->begin(st) : -1;
+                int32_t *S_twin = twin ? twin->scr->S.p : pair ? scr.S2.p : nullptr;
+                SCDE_CUDA(launch_bound_pass(q, g0, n_pos, ps, ctx->n_sm, scr.S.p, S_twin, st));
+                const PruneSide s0{scr.SR.p, scr.S.p, scr.zb.p, ps};
+                const PruneSide s1 = twin ? PruneSide{twin->scr->SR.p, S_twin, twin->scr->zb.p, ps}
+                                          : PruneSide{scr.SR2.p, S_twin, scr.zb.p, ps + 1};
+                SCDE_CUDA(launch_prune_items(q, g0, n_pos, s0, (twin || pair) ? &s1 : nullptr, scr.live.p, scr.items.p,
+                                             scr.n_live.p, prune_stats, st));
+                if (tm) tm->end(SCDE_B200_T_BOUND, e0, st, 3);
+                q.items = scr.items.p;
+                q.n_live = scr.n_live.p;
+            }
+            e0 = tm ? tm->begin(st) : -1;
             SCDE_CUDA(launch_contract_i8_pass(q, g0, n_pos, ps, ctx->n_sm, scr.T.p, st));
+            q.items = nullptr;
+            q.n_live = nullptr;
             if (pair) {
                 q.W8_twin = nullptr;
                 q.t_twin = nullptr;
             }
+            const uint8_t *live = prune ? scr.live.p : nullptr;
             if (tm) tm->end(SCDE_B200_T_CONTRACT, e0, st, 1);
             e0 = tm ? tm->begin(st) : -1;
-            SCDE_CUDA(launch_softmax_i8(q, g0, n_pos, ps, scr.T.p, scr.SR.p, scr.spart.p, ctx->n_sm, st));
+            SCDE_CUDA(launch_softmax_i8(q, g0, n_pos, ps, scr.T.p, scr.SR.p, scr.spart.p, ctx->n_sm, st, live));
             if (twin)
                 SCDE_CUDA(launch_softmax_i8(q2, g0, n_pos, ps, twin->scr->T.p, twin->scr->SR.p, twin->scr->spart.p,
-                                            ctx->n_sm, st));
+                                            ctx->n_sm, st, live));
             if (pair) {
-                SCDE_CUDA(launch_softmax_i8(q, g0, n_pos, ps + 1, scr.T2.p, scr.SR2.p, scr.spart.p, ctx->n_sm, st));
+                SCDE_CUDA(launch_softmax_i8(q, g0, n_pos, ps + 1, scr.T2.p, scr.SR2.p, scr.spart.p, ctx->n_sm, st, live));
                 ++ps;
             }
             if (tm) tm->end(SCDE_B200_T_SOFTMAX, e0, st, (twin || pair) ? 4 : 2);
@@ -589,7 +646,7 @@ int run_joint(scde_b200_ctx *ctx, ContractChoice k, const LpTable &t, const int3
     SCDE_CUDA(scr.lst_cell.ensure((size_t)t.n_genes * ld_lst));
     SCDE_CUDA(scr.lst_len.ensure((size_t)t.n_genes));
     SCDE_CUDA(scr.order.ensure((size_t)t.n_genes));
-    SCDE_CUDA(scr.total.ensure(1));
+    SCDE_CUDA(scr.total.ensure(5));
     const bool zb = t.zero_base && t.ld <= KP_TILED;
     if (zb) {
         SCDE_CUDA(scr.Z.ensure(S * z_set));
@@ -642,7 +699,8 @@ int run_joint(scde_b200_ctx *ctx, ContractChoice k, const LpTable &t, const int3
         return contract_joint_fp64(ctx, k.kernel, t, lists, scr, zb ? scr.Z.p : nullptr, n_w_rows, n_boot, sets, scale,
                                    jp_dev, ld_jp, tm);
     return contract_joint_i8(ctx, t, lists, scr, n_w_rows, n_boot, sets, scale, jp_dev, ld_jp, hot_rank, status,
-                             tw ? twin : nullptr, tm);
+                             tw ? twin : nullptr, tm, t.has_bounds && ctx->opt.prune_pieces && n_list >= PRUNE_MIN_CELLS,
+                             count_entries ? scr.total.p + 1 : nullptr);
 }
 
 // The tcgen05 status words words[0, n) once the stream has drained, copied to host[0, n).  Bits: 1 a multiplicity above
@@ -860,9 +918,13 @@ int collect_stats(StageTimer &tm, const DiffWorkspace *ws, scde_b200_stats *stat
     if (!stats) return SCDE_B200_OK;
     tm.collect(stats);
     stats->table_rows = ws->table.n_rows;
-    unsigned long long tot = 0;
-    SCDE_CUDA(cudaMemcpy(&tot, ws->scr.total.p, sizeof(tot), cudaMemcpyDeviceToHost));
-    stats->contract_cells = (int64_t)tot;
+    unsigned long long tot[5] = {0, 0, 0, 0, 0};
+    SCDE_CUDA(cudaMemcpy(tot, ws->scr.total.p, sizeof(tot), cudaMemcpyDeviceToHost));
+    stats->contract_cells = (int64_t)tot[0];
+    stats->prune_items = (int64_t)tot[1];
+    stats->prune_live = (int64_t)tot[2];
+    stats->prune_work = (int64_t)tot[3];
+    stats->prune_live_work = (int64_t)tot[4];
     return SCDE_B200_OK;
 }
 
@@ -1036,6 +1098,10 @@ int on_shards(int n, const std::vector<scde_b200_ctx *> &devs, F f, std::vector<
             }
             stats->table_rows += (*sst)[i].table_rows;
             stats->contract_cells += (*sst)[i].contract_cells;
+            stats->prune_items += (*sst)[i].prune_items;
+            stats->prune_live += (*sst)[i].prune_live;
+            stats->prune_work += (*sst)[i].prune_work;
+            stats->prune_live_work += (*sst)[i].prune_live_work;
         }
     }
     return SCDE_B200_OK;
@@ -1244,6 +1310,15 @@ int scde_b200_probe_table(scde_b200_ctx *ctx, const double *models, int32_t n_ce
                           const int32_t *ucl_offsets, const double *magnitudes, int32_t n_grid, int32_t local_theta,
                           int32_t square_logit_conc, int32_t n_cells_for_clamp, int8_t *q_out, uint32_t *row_range_out,
                           int32_t *zero_row_out, int32_t *based_out, double *zero_rows_out) {
+    return scde_b200_probe_table_bounds(ctx, models, n_cells, ucl_flat, ucl_offsets, magnitudes, n_grid, local_theta,
+                                        square_logit_conc, n_cells_for_clamp, q_out, row_range_out, zero_row_out, based_out,
+                                        zero_rows_out, nullptr);
+}
+
+int scde_b200_probe_table_bounds(scde_b200_ctx *ctx, const double *models, int32_t n_cells, const int32_t *ucl_flat,
+                                 const int32_t *ucl_offsets, const double *magnitudes, int32_t n_grid, int32_t local_theta,
+                                 int32_t square_logit_conc, int32_t n_cells_for_clamp, int8_t *q_out, uint32_t *row_range_out,
+                                 int32_t *zero_row_out, int32_t *based_out, double *zero_rows_out, int8_t *qbound_out) {
     CHECK_CTX(ctx);
     if (!models || !ucl_flat || !ucl_offsets || !magnitudes || !q_out || !row_range_out || !zero_row_out || !based_out ||
         !zero_rows_out || n_cells < 1 || n_grid < 1 || n_cells_for_clamp < 1 || ucl_offsets[0] != 0) {
@@ -1279,6 +1354,7 @@ int scde_b200_probe_table(scde_b200_ctx *ctx, const double *models, int32_t n_ce
     t.fast_theta = !local_theta && theta_all_regular(models, n_cells, n_cells);
     t.zero_base = true;
     t.want_q = true;
+    t.want_bounds = qbound_out != nullptr;
     t.want_modes = false;
     DBuf<double> d_models, d_mag;
     TRY(upload(d_models, models, (size_t)n_cells * 12, st));
@@ -1291,6 +1367,7 @@ int scde_b200_probe_table(scde_b200_ctx *ctx, const double *models, int32_t n_ce
         return SCDE_B200_EINVAL;
     }
     SCDE_CUDA(cudaMemcpyAsync(q_out, t.q.p, (size_t)t.n_rows * q_row_bytes(n_grid), cudaMemcpyDeviceToHost, st));
+    if (qbound_out && t.has_bounds) SCDE_CUDA(cudaMemcpyAsync(qbound_out, t.qb.p, (size_t)t.n_rows * Q_BW, cudaMemcpyDeviceToHost, st));
     SCDE_CUDA(cudaMemcpyAsync(row_range_out, t.qrange.p, sizeof(uint32_t) * t.n_rows, cudaMemcpyDeviceToHost, st));
     SCDE_CUDA(cudaMemcpyAsync(zero_row_out, t.zero_row.p, sizeof(int32_t) * n_cells, cudaMemcpyDeviceToHost, st));
     SCDE_CUDA(cudaMemcpyAsync(based_out, t.based.p, sizeof(int32_t) * n_cells, cudaMemcpyDeviceToHost, st));
@@ -1838,7 +1915,20 @@ int scde_b200_probe_contract_i8(scde_b200_ctx *ctx, const int8_t *qtable, int32_
                                 const uint32_t *row_range, const int8_t *w8, int32_t n_w_rows, const int32_t *lst_row,
                                 const int32_t *lst_cell, const int32_t *lst_len, int32_t n_genes, int32_t ld_lst,
                                 double *t_out, int32_t *flags_out) {
+    return scde_b200_probe_prune_i8(ctx, qtable, n_rows, n_grid, row_range, nullptr, nullptr, w8, n_w_rows, lst_row, lst_cell,
+                                    lst_len, n_genes, ld_lst, t_out, nullptr, nullptr, nullptr, nullptr, flags_out);
+}
+
+int scde_b200_probe_prune_i8(scde_b200_ctx *ctx, const int8_t *qtable, int32_t n_rows, int32_t n_grid,
+                             const uint32_t *row_range, const int8_t *qbound, const double *z, const int8_t *w8,
+                             int32_t n_w_rows, const int32_t *lst_row, const int32_t *lst_cell, const int32_t *lst_len,
+                             int32_t n_genes, int32_t ld_lst, double *t_out, double *lb_out, double *ub_out,
+                             uint8_t *live_out, double *exp_out, int32_t *flags_out) {
     CHECK_CTX(ctx);
+    if (qbound && (!lb_out || !ub_out || !live_out)) {
+        set_error("probe_prune_i8: bad arguments");
+        return SCDE_B200_EINVAL;
+    }
     if (!qtable || !w8 || !lst_row || !lst_cell || !lst_len || !t_out || n_rows < 1 || n_genes < 1 || n_w_rows < 1 ||
         !contract_i8_supported(n_grid, KP_TILED, ld_lst, 1) || n_genes > contract_tiled_max_genes()) {
         set_error("probe_contract_i8: bad arguments");
@@ -1891,9 +1981,37 @@ int scde_b200_probe_contract_i8(scde_b200_ctx *ctx, const int8_t *qtable, int32_
     q.cold_evict_first = 0;
     q.ring_stages = ctx->opt.ring_stages;
     SCDE_CUDA(launch_sentinel_ranges(q, 0, n_genes, 0, d_sr.p, st));
+    DBuf<int8_t> d_qb;
+    DBuf<double> d_z, d_zb, d_lb, d_ub;
+    DBuf<int32_t> d_s, d_items, d_nlive;
+    DBuf<uint8_t> d_live;
+    if (qbound) {  // the decision of the pruned contraction, with its bounds; T itself is contracted unpruned
+        TRY(upload(d_qb, qbound, (size_t)n_rows * Q_BW, st));
+        if (z) TRY(upload(d_z, z, (size_t)WP_TILED * KP_TILED, st));
+        q.qbound = d_qb.p;
+        q.Z = z ? d_z.p : nullptr;
+        SCDE_CUDA(d_zb.ensure(prune_zb_doubles(1, WP_TILED)));
+        SCDE_CUDA(d_s.ensure(prune_bound_ints(n_genes)));
+        SCDE_CUDA(d_lb.ensure((size_t)n_genes * WP_TILED));
+        SCDE_CUDA(d_ub.ensure((size_t)n_genes * WP_TILED * 4));
+        SCDE_CUDA(d_live.ensure((size_t)n_genes));
+        SCDE_CUDA(d_items.ensure((size_t)n_genes * q_pieces(n_grid)));
+        SCDE_CUDA(d_nlive.ensure(1));
+        SCDE_CUDA(launch_z_bounds(q, 1, d_zb.p, st));
+        SCDE_CUDA(launch_bound_pass(q, 0, n_genes, 0, ctx->n_sm, d_s.p, nullptr, st));
+        SCDE_CUDA(launch_prune_items(q, 0, n_genes, PruneSide{d_sr.p, d_s.p, d_zb.p, 0}, nullptr, d_live.p, d_items.p,
+                                     d_nlive.p, nullptr, st, d_lb.p, d_ub.p));
+        q.Z = nullptr;
+    }
     SCDE_CUDA(launch_contract_i8_pass(q, 0, n_genes, 0, ctx->n_sm, d_t.p, st));
     SCDE_CUDA(launch_finalize_t(q, n_genes, d_t.p, d_sr.p, st));
     SCDE_CUDA(cudaMemcpyAsync(t_out, d_t.p, sizeof(double) * nt, cudaMemcpyDeviceToHost, st));
+    if (qbound) {
+        SCDE_CUDA(cudaMemcpyAsync(lb_out, d_lb.p, sizeof(double) * n_genes * WP_TILED, cudaMemcpyDeviceToHost, st));
+        SCDE_CUDA(cudaMemcpyAsync(ub_out, d_ub.p, sizeof(double) * n_genes * WP_TILED * 4, cudaMemcpyDeviceToHost, st));
+        SCDE_CUDA(cudaMemcpyAsync(live_out, d_live.p, n_genes, cudaMemcpyDeviceToHost, st));
+    }
+    if (exp_out) SCDE_CUDA(launch_exp_probe(exp_out, st));
     SCDE_CUDA(cudaStreamSynchronize(st));
     int32_t f = 0;
     bool rerun = false;
@@ -2405,8 +2523,8 @@ static int diff_run_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, bool chunked
     cudaStream_t st = ctx->stream;
     StageTimer &tm = j->timer;
     tm.reset();
-    SCDE_CUDA(j->ws->scr.total.ensure(1));
-    SCDE_CUDA(cudaMemsetAsync(j->ws->scr.total.p, 0, sizeof(unsigned long long), st));
+    SCDE_CUDA(j->ws->scr.total.ensure(5));
+    SCDE_CUDA(cudaMemsetAsync(j->ws->scr.total.p, 0, 5 * sizeof(unsigned long long), st));
     const int G = j->G, C = j->C, K = j->K;
     const int ld = j->ws->table.ld;
     j->ws->table.want_q = k.kernel == Contraction::I8;
@@ -2428,7 +2546,7 @@ static int diff_run_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, bool chunked
             TRY(front_chunked(ctx, j, 1, &front_done));
             if (!front_done) {  // the table is rebuilt below: row ids change, the first joint is repeated
                 joint0_done = false;
-                SCDE_CUDA(cudaMemsetAsync(j->ws->scr.total.p, 0, sizeof(unsigned long long), st));
+                SCDE_CUDA(cudaMemsetAsync(j->ws->scr.total.p, 0, 5 * sizeof(unsigned long long), st));
             }
         }
         if (!front_done && ctx->copy_stream) SCDE_CUDA(cudaStreamSynchronize(ctx->copy_stream));  // the counts must be resident
@@ -2783,8 +2901,8 @@ int shard_contrasts(DatasetShard &sh, const ContrastPlan &p, const scde_b200_con
     const int G = sh.G, K = sh.K, nc = p.n_contrasts;
     const int ld = t.ld, nout = 2 * K - 1, ldo = round_up(nout, 8), nadj = 2 * nout - 1, lda = round_up(nadj, 8);
     const int n_slots = (int)p.slot_group.size(), n_bslots = (int)p.bslot_D.size();
-    SCDE_CUDA(ws->scr.total.ensure(1));
-    SCDE_CUDA(cudaMemsetAsync(ws->scr.total.p, 0, sizeof(unsigned long long), st));
+    SCDE_CUDA(ws->scr.total.ensure(5));
+    SCDE_CUDA(cudaMemsetAsync(ws->scr.total.p, 0, 5 * sizeof(unsigned long long), st));
     const int t_all = tm.begin(st);
     TRY(ensure_rows(sh, 0, k, &tm));
     TRY(upload(sh.cells, p.cells.data(), p.cells.size(), st));

@@ -64,14 +64,15 @@ cudaError_t launch_lp_rows(const double *models, int ld_models, CellRange cr, co
                            int local_theta, double sentinel, double *table, int ld_table, int32_t *row_mode, int which,
                            const int32_t *zero_row, const int32_t *based, void *row_const, const int32_t *row_snap,
                            int write_f64, int8_t *qtable, uint32_t *row_range, cudaStream_t st, int legacy_q_rows = 0,
-                           unsigned long long *work_counter = nullptr, int zero_compact = 0);
+                           unsigned long long *work_counter = nullptr, int zero_compact = 0, int8_t *qbound = nullptr);
 // legacy_q_rows: build fixed-point-only rows with the per-element kernel the register-resident one replaced (tests)
 // work_counter: one device word the register-resident row kernel hands its row chunks out from (zeroed by the launcher;
 // required whenever that kernel is chosen, i.e. qtable != NULL with which == 2 on the constant-theta path)
 // zero_compact: `table` is the compact FP64 table (see launch_based_flags); which == 1 writes a cell's zero-count row at the
 // cell's index, which == 2 reads it there
 // write_f64 = 0: the FP64 row is not stored (table is still read for the zero-count rows); qtable != NULL: also emit the
-// row's fixed-point planes and its non-sentinel range (contract_i8.cu) -- both only on the constant-theta fast path
+// row's fixed-point planes and its non-sentinel range (contract_i8.cu) -- both only on the constant-theta fast path -- and,
+// when qbound != NULL, its bound row (Q_BW bytes per row)
 // per-row constants of the constant-theta fast path (4 doubles per row), one thread per row
 // ... and row_snap[r] = grid point where the reference's snap rule replaces mu_k by the count, or -1 (needs prep.mu)
 cudaError_t launch_row_consts(const double *models, int ld_models, const int32_t *row_off, CellRange cr,
@@ -181,10 +182,55 @@ constexpr int Q_MAX_K = 4 * Q_PW; // largest grid the kernel takes (T rows are K
 constexpr int Q_WB = 128;         // bytes per int8 W row: 104 boots + zero padding = M of the MMA
 constexpr uint32_t Q_RANGE_IRREGULAR = 0xFFFFFFFFu;
 inline int q_pieces(int K) { return (K + Q_PW - 1) / Q_PW; }
+// Bound rows (DESIGN.md 4.3, "Pruned pieces"): next to its planes every fixed-point row has Q_BW bytes of bounds on its value
+// x = 2^29 D, in units of 2^-5 nat (x / 2^24), rounded outwards: slot u < Q_UB_N holds ceil(max x / 2^24) over the row's
+// non-sentinel points of grid block [16 u, 16 u + 16) (0 when it has none), slot Q_UB_N + c floor(x / 2^24) at the sample
+// point Q_LB_STEP c + Q_LB_OFF (0 at a sentinel).  Slot i is stored as two signed radix-256 digits, bytes i and
+// Q_BSLOTS + i, so that the contraction over the drawn rows (the tcgen05 kernel with one 128-byte piece) sums them exactly.
+constexpr int Q_BW = 128;
+constexpr int Q_BSLOTS = Q_BW / 2;
+constexpr int Q_UB_PTS = 16, Q_UB_N = KP_TILED / Q_UB_PTS;  // 26 blocks
+constexpr int Q_LB_STEP = 12, Q_LB_OFF = 6, Q_LB_N = 35;     // samples 6, 18, .., 414
+static_assert(Q_UB_N + Q_LB_N <= Q_BSLOTS && Q_LB_STEP * (Q_LB_N - 1) + Q_LB_OFF < KP_TILED, "bound row layout");
+// a row's bound slot as the two digits of its bound row
+__host__ __device__ inline void q_bound_store(int8_t *brow, int slot, int v) {
+    const int lo = (int)(int8_t)(v & 0xFF);
+    brow[slot] = (int8_t)lo;
+    brow[Q_BSLOTS + slot] = (int8_t)((v - lo) >> 8);
+}
 inline int q_row_bytes(int K) { return q_pieces(K) * Q_PIECE; }
+#ifdef __CUDACC__
+// the bound row of a fixed-point row from its planes (q: [piece][plane][102], generic address) and its non-sentinel range;
+// lanes l, l + LW, .. of a group of LW lanes take the slots.  (The register-resident row kernel computes the same values
+// from its registers: lp_table.cu.)
+__device__ inline long long q_value_at(const int8_t *q, int k) {
+    const int pc = k / Q_PW, i = k - pc * Q_PW;
+    long long x = 0;
+#pragma unroll
+    for (int pl = Q_NV - 1; pl >= 0; --pl) x = x * 256 + q[pc * Q_PIECE + pl * Q_PW + i];
+    return x;
+}
+__device__ inline void q_bound_row(const int8_t *q, int K, uint32_t range, int8_t *brow, int l, int LW) {
+    int klo = 0, khi = K - 1;
+    if (range != Q_RANGE_IRREGULAR) {
+        klo = (int)(range & 0xFFFFu);
+        khi = (int)(range >> 16);
+    }
+    for (int u = l; u < Q_UB_N; u += LW) {
+        long long m = INT64_MIN;
+        for (int k = max(u * Q_UB_PTS, klo); k < (u + 1) * Q_UB_PTS && k <= khi; ++k) m = max(m, q_value_at(q, k));
+        // ceil(x / 2^24) by an arithmetic shift
+        q_bound_store(brow, u, m == INT64_MIN ? 0 : (int)((m + ((1ll << 24) - 1)) >> 24));
+    }
+    for (int c = l; c < Q_LB_N; c += LW) {
+        const int k = Q_LB_STEP * c + Q_LB_OFF;
+        q_bound_store(brow, Q_UB_N + c, k < K ? (int)(q_value_at(q, k) >> 24) : 0);
+    }
+}
+#endif
 // planes and ranges of every row of an FP64 table (ld_table >= K); one warp per row
 cudaError_t launch_quantize_rows(const double *table, int ld_table, int K, int64_t n_rows, int8_t *qtable,
-                                 uint32_t *row_range, cudaStream_t st);
+                                 uint32_t *row_range, int8_t *qbound, cudaStream_t st);
 // W8[pass][row][128] = (int8) W[pass][row][0..104); *flag |= 1 if a multiplicity exceeds 127
 cudaError_t launch_w_to_i8(const double *W, int n_w_rows, int n_boot, int8_t *W8, int32_t *flag, cudaStream_t st);
 struct ContractI8Args {
@@ -216,6 +262,9 @@ struct ContractI8Args {
                        // rows are loaded with the L2 evict_last policy, the others evict_first.  < 0: no hints
     int cold_evict_first;  // with hot_rank >= 0: 1 = the other rows are loaded evict_first, 0 = without a priority
     int ring_stages;       // 0 / 10: the full 10-stage ring (200 KB in flight per SM); 7 or 8: a shallower one
+    const int8_t *qbound;  // the table's bound rows [rows][Q_BW] (launch_bound_pass)
+    const int32_t *items;  // launch_contract_i8_pass: contract only the live items, items[0 .. *n_live) (launch_prune_items);
+    const int32_t *n_live; // NULL = every item
 };
 constexpr int32_t LIST_HOT_BIT = 1 << 30;  // in GeneLists::cell (W row ids are < 65536)
 // n_draws: draws per randomization (the plane sums are combined pairwise in 32 bits: 257 * 128 * draws < 2^31)
@@ -233,8 +282,34 @@ cudaError_t launch_contract_i8_pass(const ContractI8Args &a, int g0, int n_pos, 
 // the rest of the gene: a.jp[gene][k] (+)= sum_b softmax_k(2^-29 T + Z)[k] / a.scale with the sentinel ranges `sr` (what
 // launch_sentinel_ranges wrote; required when a.row_range != NULL); part_scratch: softmax_i8_scratch_doubles(n_pos)
 size_t softmax_i8_scratch_doubles(int n_pos);
+// live (NULL: every piece): the pieces launch_prune_items left live, whose T tiles are the only ones written
 cudaError_t launch_softmax_i8(const ContractI8Args &a, int g0, int n_pos, int pass, const double *t_scratch, const uint32_t *sr,
-                              double *part_scratch, int n_sm, cudaStream_t st);
+                              double *part_scratch, int n_sm, cudaStream_t st, const uint8_t *live = nullptr);
+// ---- pruning (DESIGN.md 4.3): (gene, piece) items whose grid points the soft-max cannot see are not contracted
+// zb: prune_zb_doubles() doubles, the Z extrema of every (set, pass, boot) of the joint (a.Z, a.n_boot, a.K), once per joint
+size_t prune_zb_doubles(int n_sets, int n_boot);
+cudaError_t launch_z_bounds(const ContractI8Args &a, int n_sets, double *zb, cudaStream_t st);
+// S[n_pos][104][Q_BW] = the sums of the drawn rows' bound rows (a.qbound) of genes order[g0 ..), boots of `pass` -- the
+// contraction kernel with one Q_BW-byte piece; S_twin: the twin joint's (a.W8_twin), or NULL.  prune_bound_ints(n_pos) ints.
+size_t prune_bound_ints(int n_pos);
+cudaError_t launch_bound_pass(const ContractI8Args &a, int g0, int n_pos, int pass, int n_sm, int32_t *S, int32_t *S_twin,
+                              cudaStream_t st);
+// one joint's side of the decision: its sentinel ranges and bound sums of one launch, its Z extrema (first set, pass 0)
+struct PruneSide {
+    const uint32_t *sr;
+    const int32_t *S;
+    const double *zb;
+    int pass;
+};
+// live[pos] = the pieces not proven invisible for every boot of s0 (and of s1: a twin launch, where an item is contracted for
+// both joints); items / *n_live = the live items in launch order for launch_contract_i8_pass; stats (or NULL) [0] += items,
+// [1] += live items, [2] / [3] += the same weighted by the gene's list length.  live: n_pos bytes, items: n_pos *
+// q_pieces(K) ints.  lb_out [n_pos][104] / ub_out [n_pos][104][4] (tests, or NULL): s0's bounds (prune_decide_kernel).
+cudaError_t launch_prune_items(const ContractI8Args &a, int g0, int n_pos, const PruneSide &s0, const PruneSide *s1,
+                               uint8_t *live, int32_t *items, int32_t *n_live, unsigned long long *stats, cudaStream_t st,
+                               double *lb_out = nullptr, double *ub_out = nullptr);
+// tests: out_host[0..3) = exp_nonpos(-745), (-746), (-747) on the device (synchronous on st's completion of the copy)
+cudaError_t launch_exp_probe(double *out_host, cudaStream_t st);
 // tests: turns the integer tiles in t_scratch into FP64 T (a.sentinel outside the ranges, no zero-count base), in place
 cudaError_t launch_finalize_t(const ContractI8Args &a, int n_pos, double *t_scratch, const uint32_t *sr, cudaStream_t st);
 

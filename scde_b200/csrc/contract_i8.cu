@@ -96,6 +96,8 @@ struct I8Params {
                          // neighbouring CTAs gather the same table rows at the same time and the second read is an L2 hit
     int piece_major;     // item order: 0 = (gene, piece) with the piece fastest, 1 = (piece, gene) with the gene fastest
     int cold_evict_first;  // HINT kernels: rows without the hot bit are loaded evict_first (else without a hint)
+    const int32_t *items;  // pruned launch: the codes (item numbers of the order above) of the live items, *n_live of
+    const int32_t *n_live; // them, written on the device by prune_compact_kernel; NULL = every item
 };
 
 __device__ __forceinline__ bool wait_or_abort(I8Smem &sm, uint64_t *bar, uint32_t parity) {
@@ -119,9 +121,13 @@ __device__ __forceinline__ bool wait_or_abort(I8Smem &sm, uint64_t *bar, uint32_
 struct Item {
     int pos, piece;
 };
+__device__ __forceinline__ int item_code(const I8Params &p, int item) {
+    item >>= p.twin;  // twin launch: bit 0 of the item selects the joint
+    return p.items ? __ldg(p.items + item) : item;
+}
 __device__ __forceinline__ Item decode_item(const I8Params &p, int item) {
     Item it;
-    item >>= p.twin;  // twin launch: bit 0 of the item selects the joint
+    item = item_code(p, item);
     if (p.piece_major) {
         it.piece = item / p.n_pos;
         it.pos = item - it.piece * p.n_pos;
@@ -132,7 +138,7 @@ __device__ __forceinline__ Item decode_item(const I8Params &p, int item) {
     return it;
 }
 __device__ __forceinline__ int64_t item_gene(const I8Params &p, int item) {
-    item >>= p.twin;
+    item = item_code(p, item);
     const int pos = p.piece_major ? item % p.n_pos : item / p.n_pieces;
     return p.order ? p.order[pos] : pos;
 }
@@ -163,7 +169,8 @@ __device__ __forceinline__ void cp_async16_hint_at(uint32_t dst_smem, const void
 // HINT: list entries carry LIST_HOT_BIT in `cell` when the row is one of the first few of its cell (a small count: such a
 // row is shared by thousands of genes); its pieces are loaded with the L2 evict_last policy, the others evict_first (or
 // unhinted), so that the stream of rows that are used once does not push the shared ones out of the L2.
-template <int Q_PGROUPS, bool HINT, int NS>
+// BOUND: the bound pass -- one Q_BW-byte piece per row (p.qtable = the bound rows), one 128-byte run per entry.
+template <int Q_PGROUPS, bool HINT, int NS, bool BOUND>
 __device__ __forceinline__ void run_producer(const I8Params &p, I8Smem &sm, uint32_t stage0, int n_items, int warp, int lane) {
     uint64_t pol_hot = 0, pol_cold = 0;
     if (HINT) {
@@ -197,7 +204,7 @@ __device__ __forceinline__ void run_producer(const I8Params &p, I8Smem &sm, uint
             len_n = p.lst_len[gene_n];
             if (p.gene_set) wset_n = p.gene_set[gene_n] * p.set_w8;
         }
-        const int8_t *qbase = p.qtable + (int64_t)it.piece * Q_PIECE + l7 * 16;
+        const int8_t *qbase = p.qtable + (BOUND ? 0 : (int64_t)it.piece * Q_PIECE) + l7 * 16;
         const int8_t *wbase = ((p.twin && (item & 1)) ? p.W8b : p.W8) + l7 * 16 + wset;
         const int32_t *lrow = p.lst_row + gene * p.ld_lst + kg * 8 + l3;
         const int32_t *lcell = p.lst_cell + gene * p.ld_lst + kg * 8 + l3;
@@ -235,7 +242,12 @@ __device__ __forceinline__ void run_producer(const I8Params &p, I8Smem &sm, uint
                     const int8_t *w0 = wbase + (int64_t)(cel0 & ~LIST_HOT_BIT) * Q_WB;
                     const int8_t *w1 = wbase + (int64_t)(cel1 & ~LIST_HOT_BIT) * Q_WB;
                     if (fill > 0 && !wait_or_abort(sm, &sm.empty[slot], (fill - 1) & 1u)) return;
-                    if (HINT) {
+                    if (BOUND) {
+                        cp_async16_at<0, 0>(sB0, src0);
+                        cp_async16_at<0, 0>(sB1, src1);
+                        cp_async16_at<0, 0>(sA + d0, w0);
+                        cp_async16_at<0, 0>(sA + d1, w1);
+                    } else if (HINT) {
                         const uint64_t pol0 = (cel0 & LIST_HOT_BIT) ? pol_hot : pol_cold;
                         const uint64_t pol1 = (cel1 & LIST_HOT_BIT) ? pol_hot : pol_cold;
                         cp_async16_hint_at<0, 0>(sB0, src0, pol0);
@@ -284,9 +296,9 @@ __device__ __forceinline__ void run_producer(const I8Params &p, I8Smem &sm, uint
 }
 
 // ---- MMA issuer (one thread) ------------------------------------------------------------------------------------------
-template <int NS>
+template <int NS, bool BOUND>
 __device__ __forceinline__ void run_mma(const I8Params &p, I8Smem &sm, uint32_t stage0, uint32_t tmem, int n_items) {
-    const uint32_t idesc = umma_idesc_s8_mn(128, 256);
+    const uint32_t idesc = umma_idesc_s8_mn(128, BOUND ? Q_BW : 256);
     int slot = 0;
     uint32_t fill = 0, n_done = 0;
     int item = blockIdx.x;
@@ -308,7 +320,7 @@ __device__ __forceinline__ void run_mma(const I8Params &p, I8Smem &sm, uint32_t 
             const uint32_t sB = sA + Q_A_BYTES;
             const uint64_t da = umma_desc_sw128(sA, 4096u, 1024u);
             umma_s8(tmem, da, umma_desc_sw128(sB, 4096u, 1024u), idesc, s > 0);                      // runs 0, 1
-            umma_s8(tmem + 256u, da, umma_desc_sw128(sB + 2u * 4096u, 4096u, 1024u), idesc, s > 0);  // runs 2, 3
+            if (!BOUND) umma_s8(tmem + 256u, da, umma_desc_sw128(sB + 2u * 4096u, 4096u, 1024u), idesc, s > 0);  // runs 2, 3
             umma_commit(&sm.empty[slot]);  // frees the slot once these MMAs have read it
             if (++slot == NS) {
                 slot = 0;
@@ -404,7 +416,40 @@ __device__ __forceinline__ void run_epilogue(const I8Params &p, I8Smem &sm, uint
     }
 }
 
-template <int Q_PGROUPS, bool HINT, int NS>
+// bound pass: the 128 int32 sums of a (gene, boot), stored as they are (p.T / p.Tb: [n_pos][104][Q_BW]); warp e reads the
+// lanes of quarter e & 3 and the columns 64 (e >> 2) .. + 63
+__device__ __forceinline__ void run_bound_epilogue(const I8Params &p, I8Smem &sm, uint32_t tmem, int n_items, int ewarp, int lane) {
+    const int qd = ewarp & 3, half = ewarp >> 2;
+    const uint32_t tcol = tmem + ((uint32_t)(qd * 32) << 16) + (uint32_t)(half * 64);
+    const int boot = qd * 32 + lane;
+    uint32_t n_done = 0;
+    for (int item = blockIdx.x; item < n_items; item += gridDim.x, ++n_done) {
+        const int pos = item >> p.twin;
+        const bool empty_list = p.lst_len[p.order ? p.order[pos] : pos] <= 0;
+        while (!mbar_try_wait(&sm.acc_full, n_done & 1u)) {
+            __nanosleep(200);
+            if (sm.abort) return;
+        }
+        tc_fence_after_sync();
+        int4 *dst = reinterpret_cast<int4 *>(reinterpret_cast<int32_t *>((p.twin && (item & 1)) ? p.Tb : p.T) +
+                                             ((int64_t)pos * WP_TILED + boot) * Q_BW + half * 64);
+        for (int c = 0; c < 64; c += 8) {
+            uint32_t r[8] = {0u, 0u, 0u, 0u, 0u, 0u, 0u, 0u};
+            if (!empty_list) {
+                tmem_ld_32x32b_x8(tcol + (uint32_t)c, r);
+                tmem_wait_ld();
+            }
+            if (boot < p.n_boot) {
+                dst[c / 4] = make_int4((int)r[0], (int)r[1], (int)r[2], (int)r[3]);
+                dst[c / 4 + 1] = make_int4((int)r[4], (int)r[5], (int)r[6], (int)r[7]);
+            }
+        }
+        tc_fence_before_sync();
+        mbar_arrive(&sm.acc_empty);
+    }
+}
+
+template <int Q_PGROUPS, bool HINT, int NS, bool BOUND>
 __global__ void __launch_bounds__(q_threads(Q_PGROUPS), 1) contract_i8_kernel(const I8Params p) {
     static_assert(NS >= 2 && NS <= Q_NS, "ring depth");
     constexpr int Q_PRODUCER_WARPS = 4 * Q_PGROUPS;
@@ -430,14 +475,17 @@ __global__ void __launch_bounds__(q_threads(Q_PGROUPS), 1) contract_i8_kernel(co
     __syncthreads();
     tc_fence_after_sync();
     const uint32_t tmem = sm.tmem_base;
-    const int n_items = (p.n_pos * p.n_pieces) << p.twin;
+    const int n_items = (p.items ? *p.n_live : p.n_pos * p.n_pieces) << p.twin;
 
     if (warp < Q_PRODUCER_WARPS)
-        run_producer<Q_PGROUPS, HINT, NS>(p, sm, stage0, n_items, warp, lane);
-    else if (warp < Q_PRODUCER_WARPS + Q_EPILOGUE_WARPS)
-        run_epilogue(p, sm, xbuf, tmem, n_items, warp - Q_PRODUCER_WARPS, lane);
-    else if (lane == 0)
-        run_mma<NS>(p, sm, stage0, tmem, n_items);
+        run_producer<Q_PGROUPS, HINT, NS, BOUND>(p, sm, stage0, n_items, warp, lane);
+    else if (warp < Q_PRODUCER_WARPS + Q_EPILOGUE_WARPS) {
+        if (BOUND)
+            run_bound_epilogue(p, sm, tmem, n_items, warp - Q_PRODUCER_WARPS, lane);
+        else
+            run_epilogue(p, sm, xbuf, tmem, n_items, warp - Q_PRODUCER_WARPS, lane);
+    } else if (lane == 0)
+        run_mma<NS, BOUND>(p, sm, stage0, tmem, n_items);
 
     tc_fence_before_sync();
     __syncthreads();
@@ -555,12 +603,16 @@ static_assert(SP_GROUPS * SP_ROWS == WP_TILED && SP_ROWS * 32 == KP_TILED, "13 w
 // accumulators per lane in ascending boot order.
 // SETS (several draw sets, DESIGN.md "Draw sets"): each gene reads the Z rows of its own set, gene_set[gene] * set_z doubles
 // after Z, from global memory (L2) instead of shared memory -- the same values in the same order, so the same result.
+// live (pruned launches, else NULL): bit p of live[pos] = piece p of the gene was contracted.  The points of the other
+// pieces are neither loaded (their T tiles were not written) nor candidates: prune_decide_kernel proved them more than
+// 746 nats below the row maximum for every boot, where exp_nonpos is exactly 0 -- m, sum, amask and acc are unchanged.
 constexpr int SW_WARPS = 8;
-template <bool SETS>
+// LIVE: the instance of pruned launches (live != NULL); the other one is the kernel as it was before pruning.
+template <bool SETS, bool LIVE>
 __global__ void __launch_bounds__(SW_WARPS * 32, 2)
 softmax_i8_warp_kernel(const long long *__restrict__ T, const double *__restrict__ Z, const uint32_t *__restrict__ SR, int K,
                        int n_boot_pass, double scale, double *__restrict__ part, int n_pos, const int32_t *__restrict__ order,
-                       const int32_t *__restrict__ gene_set, int64_t set_z) {
+                       const int32_t *__restrict__ gene_set, int64_t set_z, const uint8_t *__restrict__ live) {
     constexpr int NJ = KP_TILED / 32;
     extern __shared__ double s_z[];  // [SP_ROWS][KP_TILED] (one set only)
     const int group = blockIdx.x % SP_GROUPS, batch = blockIdx.x / SP_GROUPS, n_batch = gridDim.x / SP_GROUPS;
@@ -582,10 +634,17 @@ softmax_i8_warp_kernel(const long long *__restrict__ T, const double *__restrict
         const uint32_t sr_l = (SR && lane < SP_ROWS) ? SR[(int64_t)pos * Q_WB + b0 + lane] : 0xFFFF0000u;
         const double *zg = s_z;
         if (SETS) zg = Z + gene_set[order ? order[pos] : pos] * set_z + (int64_t)b0 * KP_TILED;
+        uint32_t lm = (1u << NJ) - 1u;  // bit j: stretch j of this lane lies in a contracted piece
+        if (LIVE) {
+            const uint32_t pm = live[pos];
+            lm = 0u;
+#pragma unroll
+            for (int j = 0; j < NJ; ++j) lm |= ((pm >> ((lane + 32 * j) / Q_PW)) & 1u) << j;
+        }
         long long nxt[NJ];
         if (nb > 0) {
 #pragma unroll
-            for (int j = 0; j < NJ; ++j) nxt[j] = __ldcs(rows + 32 * j);
+            for (int j = 0; j < NJ; ++j) nxt[j] = (lm >> j) & 1u ? __ldcs(rows + 32 * j) : 0ll;
         }
         for (int bi = 0; bi < nb; ++bi) {
             long long cur[NJ];
@@ -594,7 +653,7 @@ softmax_i8_warp_kernel(const long long *__restrict__ T, const double *__restrict
             if (bi + 1 < nb) {
                 const long long *r2 = rows + (int64_t)(bi + 1) * KP_TILED;
 #pragma unroll
-                for (int j = 0; j < NJ; ++j) nxt[j] = __ldcs(r2 + 32 * j);
+                for (int j = 0; j < NJ; ++j) nxt[j] = (lm >> j) & 1u ? __ldcs(r2 + 32 * j) : 0ll;
             }
             const uint32_t sr = __shfl_sync(0xffffffffu, sr_l, bi);
             const int klo = (int)(sr & 0xFFFFu), span = min((int)(sr >> 16), K - 1) - klo;  // admissible: klo .. klo + span
@@ -605,7 +664,7 @@ softmax_i8_warp_kernel(const long long *__restrict__ T, const double *__restrict
                 const int k = lane + 32 * j;
                 // some drawn row is "log 0" outside the range: the reference's T is a multiple of the sentinel there
                 const double t = fma((double)cur[j], q, zr[32 * j]);
-                v[j] = (unsigned)(k - klo) <= (unsigned)span && span >= 0 ? t : -INFINITY;
+                v[j] = (unsigned)(k - klo) <= (unsigned)span && span >= 0 && ((lm >> j) & 1u) ? t : -INFINITY;
                 m = v[j] > m ? v[j] : m;
             }
 #pragma unroll
@@ -667,11 +726,171 @@ __global__ void finalize_t_kernel(long long *__restrict__ T, const uint32_t *__r
 }
 
 // ------------------------------------------------------------------------------------------------
+// Pruning (DESIGN.md 4.3).  For a (gene, boot) with sentinel range [klo, khi] and S = the bound pass's sums over the drawn
+// rows (units of 2^-5 nat, rounded outwards row by row, so exact bounds on the integer T):
+//   LB = max over the samples k_c in [klo, khi] of Z(k_c) + S_lb[c] / 32  <=  T(k_c)  <=  the row maximum m,
+//   UB_p = max over the blocks meeting [klo, khi] and piece p of max Z over the block + S_ub[u] / 32  >=  every admissible
+//          T of piece p.
+// Piece p is dead when UB_p < LB - 747 for every real boot: its points lie more than 746 nats below m (one nat covers the
+// FP64 rounding of fma(T, 2^-29, Z) and of these sums), where the soft-max adds exactly 0.
+
+// zb[row][slot] (row = (set, pass, boot), the rows of Z): max of Z over UB block `slot`, Z at LB sample slot - Q_UB_N
+__global__ void z_bounds_kernel(const double *__restrict__ Z, int64_t n_rows, int K, double *__restrict__ zb) {
+    const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= n_rows * Q_BSLOTS) return;
+    const int64_t row = idx / Q_BSLOTS;
+    const int s = (int)(idx - row * Q_BSLOTS);
+    const double *z = Z + row * KP_TILED;
+    double v = -INFINITY;
+    if (s < Q_UB_N) {
+        for (int k = s * Q_UB_PTS; k < (s + 1) * Q_UB_PTS && k < K; ++k) v = fmax(v, Z ? z[k] : 0.0);
+    } else if (s < Q_UB_N + Q_LB_N) {
+        const int k = Q_LB_STEP * (s - Q_UB_N) + Q_LB_OFF;
+        if (k < K) v = Z ? z[k] : 0.0;
+    }
+    zb[idx] = v;
+}
+
+// one warp per gene: live[pos] = the pieces that are not dead for the boots of side 0 (and of side 1: twin launches)
+struct PruneSideDev {
+    const uint32_t *sr;
+    const int32_t *S;
+    const double *zb;
+    int n_boot;
+};
+__global__ void __launch_bounds__(256) prune_decide_kernel(PruneSideDev s0, PruneSideDev s1, int sides, const int32_t *__restrict__ order,
+                                                           const int32_t *__restrict__ gene_set, int64_t set_zb, int n_pos, int K,
+                                                           int n_pieces, uint8_t *__restrict__ live, double *__restrict__ lb_out,
+                                                           double *__restrict__ ub_out) {
+    const int pos = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (pos >= n_pos) return;
+    const int lane = threadIdx.x & 31;
+    const int64_t zoff = gene_set ? gene_set[order ? order[pos] : pos] * set_zb : 0;
+    const uint32_t all = (1u << n_pieces) - 1u;
+    uint32_t dead = all;
+    for (int side = 0; side < sides; ++side) {
+        const PruneSideDev s = side ? s1 : s0;
+        for (int b = lane; b < s.n_boot; b += 32) {
+            const uint32_t sr = s.sr ? s.sr[(int64_t)pos * Q_WB + b] : 0xFFFF0000u;
+            const int klo = (int)(sr & 0xFFFFu), khi = min((int)(sr >> 16), K - 1);
+            const int32_t *S = s.S + ((int64_t)pos * WP_TILED + b) * Q_BW;
+            const double *z = s.zb + zoff + (int64_t)b * Q_BSLOTS;
+            double lb = -INFINITY;
+            for (int c = 0; c < Q_LB_N; ++c) {
+                const int k = Q_LB_STEP * c + Q_LB_OFF;
+                if (k >= klo && k <= khi)
+                    lb = fmax(lb, z[Q_UB_N + c] + ((double)S[Q_UB_N + c] + 256.0 * S[Q_BSLOTS + Q_UB_N + c]) * (1.0 / 32.0));
+            }
+            double ub[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
+            for (int u = 0; u < Q_UB_N; ++u) {
+                const int lo = max(u * Q_UB_PTS, klo), hi = min(u * Q_UB_PTS + Q_UB_PTS - 1, khi);
+                if (lo > hi) continue;
+                const double v = z[u] + ((double)S[u] + 256.0 * S[Q_BSLOTS + u]) * (1.0 / 32.0);
+#pragma unroll
+                for (int pc = 0; pc < 4; ++pc)
+                    if (max(lo, pc * Q_PW) <= min(hi, pc * Q_PW + Q_PW - 1)) ub[pc] = fmax(ub[pc], v);
+            }
+            if (lb_out && side == 0) {  // scde_b200_probe_prune_i8
+                lb_out[(int64_t)pos * WP_TILED + b] = lb;
+                for (int pc = 0; pc < 4; ++pc) ub_out[((int64_t)pos * WP_TILED + b) * 4 + pc] = ub[pc];
+            }
+            const double thr = lb - 747.0;  // lb = -inf (no sample inside the range): nothing is dead
+            uint32_t d = 0u;
+#pragma unroll
+            for (int pc = 0; pc < 4; ++pc) d |= ub[pc] < thr ? 1u << pc : 0u;
+            dead &= d;
+        }
+    }
+    dead = __reduce_and_sync(0xffffffffu, dead);
+    if (lane == 0) live[pos] = (uint8_t)(~dead & all);
+}
+
+// items[0 .. *n_live) = the live items' codes in launch order (piece-major or gene-major, as decode_item reads them); one
+// CTA, four items per thread and round.  stats (may be NULL): [0] += items, [1] += live items, [2] += list entries over
+// the items (what the unpruned launch would gather, in entry-pieces), [3] += the same over the live items.
+constexpr int PC_THREADS = 1024;
+__global__ void __launch_bounds__(PC_THREADS) prune_compact_kernel(const uint8_t *__restrict__ live, int n_pos, int n_pieces,
+                                                                   int piece_major, const int32_t *__restrict__ order,
+                                                                   const int32_t *__restrict__ lst_len, int32_t *__restrict__ items,
+                                                                   int32_t *__restrict__ n_live, unsigned long long *stats) {
+    __shared__ int wsum[PC_THREADS / 32];
+    unsigned long long work = 0, live_work = 0;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int n = n_pos * n_pieces;
+    int base = 0;
+    for (int i0 = 0; i0 < n; i0 += 4 * PC_THREADS) {
+        uint32_t f = 0u;
+        int c = 0;
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+            const int i = i0 + 4 * threadIdx.x + e;
+            if (i < n) {
+                const int piece = piece_major ? i / n_pos : i % n_pieces;
+                const int pos = piece_major ? i - piece * n_pos : i / n_pieces;
+                const unsigned long long len = stats ? (unsigned long long)max(lst_len[order ? order[pos] : pos], 0) : 0ull;
+                work += len;
+                if ((live[pos] >> piece) & 1u) {
+                    f |= 1u << e;
+                    ++c;
+                    live_work += len;
+                }
+            }
+        }
+        int x = c;  // inclusive scan over the warp
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int y = __shfl_up_sync(0xffffffffu, x, o);
+            if (lane >= o) x += y;
+        }
+        if (lane == 31) wsum[warp] = x;
+        __syncthreads();
+        if (warp == 0) {
+            int w = wsum[lane];
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const int y = __shfl_up_sync(0xffffffffu, w, o);
+                if (lane >= o) w += y;
+            }
+            wsum[lane] = w;
+        }
+        __syncthreads();
+        int off = base + (warp ? wsum[warp - 1] : 0) + x - c;
+#pragma unroll
+        for (int e = 0; e < 4; ++e)
+            if ((f >> e) & 1u) items[off++] = i0 + 4 * threadIdx.x + e;
+        base += wsum[PC_THREADS / 32 - 1];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) {
+        *n_live = base;
+        if (stats) {
+            atomicAdd(stats, (unsigned long long)n);
+            atomicAdd(stats + 1, (unsigned long long)base);
+        }
+    }
+    if (stats) {
+        work = __reduce_add_sync(0xffffffffu, (unsigned)work) + 0ull;  // < 2^32: a warp sees <= 4096 items of <= 65536 entries
+        live_work = __reduce_add_sync(0xffffffffu, (unsigned)live_work) + 0ull;
+        if (lane == 0) {
+            atomicAdd(stats + 2, work);
+            atomicAdd(stats + 3, live_work);
+        }
+    }
+}
+
+// exp_nonpos at -745, -746, -747 as softmax_i8_warp_kernel evaluates it (scde_b200_probe_prune_i8): the soft-max weight of a
+// point more than 746 nats below its row maximum must be exactly 0 for pruning to leave the result unchanged
+__global__ void exp_probe_kernel(double *out) {
+    const int i = threadIdx.x;
+    if (i < 3) out[i] = exp_nonpos(-745.0 - i);
+}
+
+// ------------------------------------------------------------------------------------------------
 // fixed-point planes and non-sentinel range of every row of an FP64 table (the general row kernel writes FP64 only; the
 // constant-theta fast kernel emits both itself, lp_table.cu): one warp per row
 __global__ void __launch_bounds__(256) quantize_rows_kernel(const double *__restrict__ table, int ld_table, int K, int64_t n_rows,
                                                             int8_t *__restrict__ qtable, int64_t ldq,
-                                                            uint32_t *__restrict__ row_range) {
+                                                            uint32_t *__restrict__ row_range, int8_t *__restrict__ qbound) {
     const int64_t row = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (row >= n_rows) return;
     const int lane = threadIdx.x & 31;
@@ -701,15 +920,17 @@ __global__ void __launch_bounds__(256) quantize_rows_kernel(const double *__rest
         kmin = min(kmin, __shfl_xor_sync(0xffffffffu, kmin, o));
         kmax = max(kmax, __shfl_xor_sync(0xffffffffu, kmax, o));
     }
-    if (lane == 0) {
-        uint32_t rr;
-        if (n_ok == 0)
-            rr = Q_RANGE_IRREGULAR;  // a row of sentinels only: let the FP64 kernel deal with it
-        else if (kmax - kmin + 1 != n_ok)
-            rr = Q_RANGE_IRREGULAR;
-        else
-            rr = (uint32_t)kmin | ((uint32_t)kmax << 16);
-        row_range[row] = rr;
+    uint32_t rr;
+    if (n_ok == 0)
+        rr = Q_RANGE_IRREGULAR;  // a row of sentinels only: let the FP64 kernel deal with it
+    else if (kmax - kmin + 1 != n_ok)
+        rr = Q_RANGE_IRREGULAR;
+    else
+        rr = (uint32_t)kmin | ((uint32_t)kmax << 16);
+    if (lane == 0) row_range[row] = rr;
+    if (qbound) {
+        __syncwarp();  // the planes the other lanes wrote
+        q_bound_row(dst, K, rr, qbound + row * Q_BW, lane, 32);
     }
 }
 
@@ -736,11 +957,11 @@ __global__ void w_to_i8_kernel(const double *__restrict__ W, int64_t n_rows_tota
 }  // namespace
 
 cudaError_t launch_quantize_rows(const double *table, int ld_table, int K, int64_t n_rows, int8_t *qtable,
-                                 uint32_t *row_range, cudaStream_t st) {
+                                 uint32_t *row_range, int8_t *qbound, cudaStream_t st) {
     if (n_rows <= 0) return cudaSuccess;
     if (K > ld_table || K > Q_MAX_K) return cudaErrorInvalidValue;
     quantize_rows_kernel<<<(unsigned)((n_rows + 7) / 8), 256, 0, st>>>(table, ld_table, K, n_rows, qtable, q_row_bytes(K),
-                                                                        row_range);
+                                                                        row_range, qbound);
     return cudaGetLastError();
 }
 
@@ -781,6 +1002,8 @@ static I8Params make_params(const ContractI8Args &a, int g0, int n_pos, int pass
     p.twin = (a.W8_twin && a.t_twin) ? 1 : 0;
     p.piece_major = a.item_order == 1;
     p.cold_evict_first = a.cold_evict_first;
+    p.items = a.items;
+    p.n_live = a.items ? a.n_live : nullptr;
     return p;
 }
 
@@ -819,24 +1042,93 @@ cudaError_t launch_contract_i8_pass(const ContractI8Args &a, int g0, int n_pos, 
         kernel<<<grid, q_threads(PG), smem, st>>>(p);
         return cudaGetLastError();
     };
-    if (a.hot_rank >= 0) return launch(contract_i8_kernel<PG, true, Q_NS>, Q_NS);
+    if (a.hot_rank >= 0) return launch(contract_i8_kernel<PG, true, Q_NS, false>, Q_NS);
     // the shallow ring leaves 69 KB of shared memory and a third of the register file to a co-resident kernel
-    if (a.ring_stages == 7) return launch(contract_i8_kernel<PG, false, 7>, 7);
-    if (a.ring_stages == 8) return launch(contract_i8_kernel<PG, false, 8>, 8);
-    return launch(contract_i8_kernel<PG, false, Q_NS>, Q_NS);
+    if (a.ring_stages == 7) return launch(contract_i8_kernel<PG, false, 7, false>, 7);
+    if (a.ring_stages == 8) return launch(contract_i8_kernel<PG, false, 8, false>, 8);
+    return launch(contract_i8_kernel<PG, false, Q_NS, false>, Q_NS);
+}
+
+size_t prune_zb_doubles(int n_sets, int n_boot) {
+    const int passes = (n_boot + WP_TILED - 1) / WP_TILED;
+    return (size_t)(n_sets > 0 ? n_sets : 1) * (passes > 0 ? passes : 1) * WP_TILED * Q_BSLOTS;
+}
+
+cudaError_t launch_z_bounds(const ContractI8Args &a, int n_sets, double *zb, cudaStream_t st) {
+    const int64_t rows = (int64_t)prune_zb_doubles(n_sets, a.n_boot) / Q_BSLOTS;
+    z_bounds_kernel<<<(unsigned)((rows * Q_BSLOTS + 255) / 256), 256, 0, st>>>(a.Z, rows, a.K, zb);
+    return cudaGetLastError();
+}
+
+size_t prune_bound_ints(int n_pos) { return (size_t)(n_pos > 0 ? n_pos : 1) * WP_TILED * Q_BW; }
+
+cudaError_t launch_bound_pass(const ContractI8Args &a, int g0, int n_pos, int pass, int n_sm, int32_t *S, int32_t *S_twin,
+                              cudaStream_t st) {
+    if (n_pos <= 0) return cudaSuccess;
+    if (!a.qbound) return cudaErrorInvalidValue;
+    constexpr int PG = 1;
+    ContractI8Args b = a;
+    b.items = nullptr;
+    b.t_twin = reinterpret_cast<double *>(S_twin);
+    I8Params p = make_params(b, g0, n_pos, pass, reinterpret_cast<double *>(S));
+    p.qtable = a.qbound;
+    p.ldq = Q_BW;
+    p.n_pieces = 1;
+    p.piece_major = 0;
+    const int n_items = n_pos << p.twin;
+    int grid = n_sm < n_items ? n_sm : n_items;
+    if (p.twin) grid &= ~1;
+    auto kernel = contract_i8_kernel<PG, false, Q_NS, true>;
+    const size_t smem = q_smem_bytes(Q_NS);
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    kernel<<<grid, q_threads(PG), smem, st>>>(p);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_prune_items(const ContractI8Args &a, int g0, int n_pos, const PruneSide &s0, const PruneSide *s1,
+                               uint8_t *live, int32_t *items, int32_t *n_live, unsigned long long *stats, cudaStream_t st,
+                               double *lb_out, double *ub_out) {
+    if (n_pos <= 0) return cudaSuccess;
+    const int32_t *order = a.lists.order ? a.lists.order + g0 : nullptr;
+    auto dev = [&](const PruneSide &s) {
+        return PruneSideDev{a.row_range ? s.sr : nullptr, s.S, s.zb + (size_t)s.pass * WP_TILED * Q_BSLOTS,
+                            (a.n_boot - s.pass * WP_TILED) < WP_TILED ? (a.n_boot - s.pass * WP_TILED) : WP_TILED};
+    };
+    const int64_t set_zb = (int64_t)prune_zb_doubles(1, a.n_boot);
+    prune_decide_kernel<<<(unsigned)((n_pos + 7) / 8), 256, 0, st>>>(dev(s0), dev(s1 ? *s1 : s0), s1 ? 2 : 1, order,
+                                                                     a.gene_set, set_zb, n_pos, a.K, q_pieces(a.K), live,
+                                                                     lb_out, ub_out);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    prune_compact_kernel<<<1, PC_THREADS, 0, st>>>(live, n_pos, q_pieces(a.K), a.item_order == 1, order, a.lists.len, items,
+                                                   n_live, stats);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_exp_probe(double *out_host, cudaStream_t st) {
+    double *d = nullptr;
+    cudaError_t e = cudaMallocAsync(&d, 3 * sizeof(double), st);
+    if (e != cudaSuccess) return e;
+    exp_probe_kernel<<<1, 32, 0, st>>>(d);
+    e = cudaGetLastError();
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out_host, d, 3 * sizeof(double), cudaMemcpyDeviceToHost, st);
+    const cudaError_t f = cudaFreeAsync(d, st);
+    return e != cudaSuccess ? e : f;
 }
 
 size_t softmax_i8_scratch_doubles(int n_pos) { return (size_t)SP_GROUPS * (n_pos > 0 ? n_pos : 1) * KP_TILED; }
 
 cudaError_t launch_softmax_i8(const ContractI8Args &a, int g0, int n_pos, int pass, const double *t_scratch, const uint32_t *sr,
-                              double *part_scratch, int n_sm, cudaStream_t st) {
+                              double *part_scratch, int n_sm, cudaStream_t st, const uint8_t *live) {
     if (n_pos <= 0) return cudaSuccess;
     if (a.row_range && !sr) return cudaErrorInvalidValue;
     const int nb = (a.n_boot - pass * WP_TILED) < WP_TILED ? (a.n_boot - pass * WP_TILED) : WP_TILED;
     const double *Z = a.Z ? a.Z + (size_t)pass * WP_TILED * KP_TILED : nullptr;
     const bool sets = a.gene_set && Z;
     const size_t smem = sets ? 0 : sizeof(double) * SP_ROWS * KP_TILED;
-    auto kernel = sets ? softmax_i8_warp_kernel<true> : softmax_i8_warp_kernel<false>;
+    auto kernel = sets ? (live ? softmax_i8_warp_kernel<true, true> : softmax_i8_warp_kernel<true, false>)
+                       : (live ? softmax_i8_warp_kernel<false, true> : softmax_i8_warp_kernel<false, false>);
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     int wb = n_sm * 2 / SP_GROUPS;  // two CTAs of eight warps per SM
@@ -844,7 +1136,8 @@ cudaError_t launch_softmax_i8(const ContractI8Args &a, int g0, int n_pos, int pa
     if (wb < 1) wb = 1;
     kernel<<<wb * SP_GROUPS, SW_WARPS * 32, smem, st>>>(reinterpret_cast<const long long *>(t_scratch), Z,
                                                         a.row_range ? sr : nullptr, a.K, nb, a.scale, part_scratch, n_pos,
-                                                        a.lists.order ? a.lists.order + g0 : nullptr, a.gene_set, a.set_z);
+                                                        a.lists.order ? a.lists.order + g0 : nullptr, a.gene_set, a.set_z,
+                                                        live);
     e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     const int64_t n = (int64_t)n_pos * KP_TILED;

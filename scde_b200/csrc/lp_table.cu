@@ -17,6 +17,7 @@
 #include "fastmath.cuh"
 #include "ptx_sm100.cuh"
 #include <cfloat>
+#include <climits>
 #include <cmath>
 #include <cstdlib>
 
@@ -503,7 +504,7 @@ lp_rows_fast_kernel(const double *__restrict__ models, int ldm, CellRange cr, co
                     const double4 *__restrict__ rowc, const int32_t *__restrict__ row_snap, CellPrep prep, int K,
                     double sentinel, double *__restrict__ table, int ld_table, int32_t *__restrict__ row_mode, int which,
                     const int32_t *__restrict__ zero_row, const int32_t *__restrict__ based, int write_f64, int zero_compact,
-                    int8_t *__restrict__ qtable, int ldq, uint32_t *__restrict__ row_range) {
+                    int8_t *__restrict__ qtable, int ldq, uint32_t *__restrict__ row_range, int8_t *__restrict__ qbound) {
     constexpr int RPW = 32 / LW;  // rows per warp
     extern __shared__ __align__(16) unsigned char s_dyn[];
     double *s_rows = reinterpret_cast<double *>(s_dyn);                                  // [ROW_WARPS * RPW][KP_TILED]
@@ -734,9 +735,9 @@ lp_rows_fast_kernel(const double *__restrict__ models, int ldm, CellRange cr, co
                 kmin = min(kmin, __shfl_xor_sync(0xffffffffu, kmin, o));
                 kmax = max(kmax, __shfl_xor_sync(0xffffffffu, kmax, o));
             }
-            if (l == 0 && valid)
-                row_range[row] = (n_ok > 0 && kmax - kmin + 1 == n_ok) ? ((uint32_t)kmin | ((uint32_t)kmax << 16))
-                                                                        : Q_RANGE_IRREGULAR;
+            const uint32_t rr = (n_ok > 0 && kmax - kmin + 1 == n_ok) ? ((uint32_t)kmin | ((uint32_t)kmax << 16)) : Q_RANGE_IRREGULAR;
+            if (l == 0 && valid) row_range[row] = rr;
+            if (qbound && valid) q_bound_row(reinterpret_cast<const int8_t *>(sq), K, rr, qbound + (size_t)row * Q_BW, l, LW);
         }
         __syncwarp();
         if (MODES && l == 0 && valid) row_mode[row] = (besti == 0x7fffffff) ? 0 : besti;
@@ -789,22 +790,41 @@ struct QrHeaders {
 struct QrCell {
     double2 E[2 * QR_MAIN + 1][32], Z[2 * QR_MAIN + 1][32];
 };
-constexpr int QR_SMEM_WARP = 4 * Q_PIECE + 2 * (int)sizeof(QrHeaders) + (int)sizeof(QrCell);
+constexpr int QR_SMEM_WARP = 4 * Q_PIECE + 2 * (int)sizeof(QrHeaders) + (int)sizeof(QrCell) + Q_BW;  // + the staged bound row
 
-template <bool FULL>  // FULL: K >= 384, every quad of the three rounds lies inside the grid
+// one slot of the staged bound row (common.cuh): its two digits
+__device__ __forceinline__ void st_bound_slot(uint32_t sb, int slot, int v) {
+    const int lo = (int)(int8_t)(v & 0xFF);
+    st_shared_u8(sb + slot, (uint32_t)lo);
+    st_shared_u8(sb + Q_BSLOTS + slot, (uint32_t)((v - lo) >> 8));
+}
+// x / 2^24 rounded up (CEIL) or down, x = rint(v 2^29) from the biased word of the digit trick below: with xb = x +
+// 0x8080808080 = 2^24 A + r, x / 2^24 = A - 0x8080 + (r - 0x808080) / 2^24
+template <bool CEIL>
+__device__ __forceinline__ int q_bound_of(uint32_t lo, uint32_t hw) {
+    const int t = (int)(__funnelshift_r(lo, hw, 24) & 0xFFFFu) - 0x8080;
+    const uint32_t r = lo & 0xFFFFFFu;
+    return CEIL ? t + (r > 0x808080u ? 1 : 0) : t - (r < 0x808080u ? 1 : 0);
+}
+
+// FULL: K >= 384, every quad of the three rounds lies inside the grid; BOUNDS: qbound != NULL (bound rows are written)
+template <bool FULL, bool BOUNDS>
 __global__ void __launch_bounds__(QR_WARPS * 32, 3)
 lp_rows_q_kernel(const double *__restrict__ models, int ldm, CellRange cr, const int32_t *__restrict__ row_off,
                  const int32_t *__restrict__ row_cell, const int32_t *__restrict__ row_x,
                  const double4 *__restrict__ rowc, const int32_t *__restrict__ row_snap, CellPrep prep, int K,
                  double sentinel, const double *__restrict__ table, int ld_table, const int32_t *__restrict__ zero_row,
                  const int32_t *__restrict__ based, int8_t *__restrict__ qtable, int ldq, uint32_t *__restrict__ row_range,
-                 unsigned long long *__restrict__ work_counter, int zero_compact) {
+                 unsigned long long *__restrict__ work_counter, int zero_compact, int8_t *__restrict__ qbound) {
     extern __shared__ __align__(16) unsigned char s_dyn[];  // [QR_WARPS][QR_SMEM_WARP]
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     uint8_t *sq = s_dyn + warp * QR_SMEM_WARP;
     QrHeaders *hdr = reinterpret_cast<QrHeaders *>(sq + 4 * Q_PIECE);
     QrCell *cell = reinterpret_cast<QrCell *>(sq + 4 * Q_PIECE + 2 * sizeof(QrHeaders));
+    uint8_t *sbnd = sq + QR_SMEM_WARP - Q_BW;  // the row's bound row (common.cuh); its unused slots stay zero
+    const uint32_t sb_addr = smem_u32(sbnd);
     for (int j = lane; j < (4 * Q_PIECE) / 16; j += 32) reinterpret_cast<uint4 *>(sq)[j] = make_uint4(0u, 0u, 0u, 0u);
+    reinterpret_cast<uint32_t *>(sbnd)[lane] = 0u;
     __syncwarp();
     const int64_t row0 = (int64_t)row_off[cr.c0];
     const int64_t row1 = min((int64_t)row_off[cr.c1], cr.row_cap);
@@ -1006,6 +1026,17 @@ lp_rows_q_kernel(const double *__restrict__ models, int ldm, CellRange cr, const
                     lo[q] = (uint32_t)yb;
                     hw[q] = (uint32_t)((unsigned long long)yb >> 32);
                 }
+                if (BOUNDS) {  // bound row: block 8 j + lane / 4 = the quads of lanes 4 (lane / 4) .. + 3; LB sample at 4 Q + 2
+                    int ub = INT_MIN;
+#pragma unroll
+                    for (int q = 0; q < 4; ++q)
+                        if ((alive >> q) & 1u) ub = max(ub, q_bound_of<true>(lo[q], hw[q]));
+                    ub = max(ub, __shfl_xor_sync(0xffffffffu, ub, 1));
+                    ub = max(ub, __shfl_xor_sync(0xffffffffu, ub, 2));
+                    if ((lane & 3) == 0) st_bound_slot(sb_addr, 8 * j + (lane >> 2), ub == INT_MIN ? 0 : ub);
+                    const int Q = lane + 32 * j;  // LB sample c at grid point 12 c + 6 = 4 (3 c + 1) + 2
+                    if (Q % 3 == 1) st_bound_slot(sb_addr, Q_UB_N + (Q - 1) / 3, (alive >> 2) & 1u ? q_bound_of<false>(lo[2], hw[2]) : 0);
+                }
                 // byte q of every plane word belongs to element q: 0xFF where it is alive (dead elements store zero digits)
                 const uint32_t am = ((alive * 0x00204081u) & 0x01010101u) * 0xFFu;
                 const uint32_t t0 = __byte_perm(lo[0], lo[1], 0x5140), t1 = __byte_perm(lo[2], lo[3], 0x5140);
@@ -1049,6 +1080,15 @@ lp_rows_q_kernel(const double *__restrict__ models, int ldm, CellRange cr, const
                 const uint32_t am = live ? 0xFFFFFFFFu : 0u;
                 const uint32_t lo = ((uint32_t)yb ^ 0x80808080u) & am, h8 = ((uint32_t)((unsigned long long)yb >> 32) ^ 0x80u) & am;
                 okmask |= live ? (1u << P) : 0u;
+                if (BOUNDS) {  // blocks 24 and 25: the single points of lanes 0..15 and 16..31
+                    const uint32_t ylo = (uint32_t)yb, yhw = (uint32_t)((unsigned long long)yb >> 32);
+                    int ub = live && tail_ok ? q_bound_of<true>(ylo, yhw) : INT_MIN;
+#pragma unroll
+                    for (int o = 1; o < 16; o <<= 1) ub = max(ub, __shfl_xor_sync(0xffffffffu, ub, o));
+                    if ((lane & 15) == 0) st_bound_slot(sb_addr, 3 * 8 + (lane >> 4), ub == INT_MIN ? 0 : ub);
+                    if (kt % Q_LB_STEP == Q_LB_OFF)
+                        st_bound_slot(sb_addr, Q_UB_N + kt / Q_LB_STEP, live && tail_ok ? q_bound_of<false>(ylo, yhw) : 0);
+                }
                 if (tail_ok) {
                     st_shared_u8(offt, lo);
                     st_shared_u8(offt + Q_PW, lo >> 8);
@@ -1068,6 +1108,7 @@ lp_rows_q_kernel(const double *__restrict__ models, int ldm, CellRange cr, const
                 } else {
                     for (int j = 0; j < ldq / 16 - lane; j += 32) dst[j] = src[j];
                 }
+                if (BOUNDS) reinterpret_cast<uint32_t *>(qbound + (size_t)row * Q_BW)[lane] = reinterpret_cast<const uint32_t *>(sbnd)[lane];
             }
             // count, first and last of the grid points that are not "log 0"; a lane's points ascend with the bit number:
             // bit b < 12 is grid point 4 lane + 128 (b >> 2) + (b & 3) = (4 lane - 96 (b >> 2)) + 32 b... written as
@@ -1136,7 +1177,7 @@ cudaError_t launch_lp_rows(const double *models, int ld_models, CellRange cr, co
                            int local_theta, double sentinel, double *table, int ld_table, int32_t *row_mode, int which,
                            const int32_t *zero_row, const int32_t *based, void *row_const, const int32_t *row_snap,
                            int write_f64, int8_t *qtable, uint32_t *row_range, cudaStream_t st, int legacy_q_rows,
-                           unsigned long long *work_counter, int zero_compact) {
+                           unsigned long long *work_counter, int zero_compact, int8_t *qbound) {
     if (cr.c1 <= cr.c0) return cudaSuccess;
     // compact FP64 table (one row per cell: its zero-count row): only the zero-count rows may be stored in FP64
     if (zero_compact && (which == 0 || (which == 2 && write_f64) || local_theta)) return cudaErrorInvalidValue;
@@ -1159,10 +1200,12 @@ cudaError_t launch_lp_rows(const double *models, int ld_models, CellRange cr, co
                 kernel<<<148 * 3, QR_WARPS * 32, smem, st>>>(models, ld_models, cr, row_off, row_cell_map, row_x,
                                                              (const double4 *)row_const, row_snap, prep, K, sentinel, table,
                                                              ld_table, zero_row, based, qtable, q_row_bytes(K), row_range,
-                                                             work_counter, zero_compact);
+                                                             work_counter, zero_compact, qtable ? qbound : nullptr);
                 return cudaGetLastError();
             };
-            return K >= 4 * 32 * QR_MAIN ? launch_q(lp_rows_q_kernel<true>) : launch_q(lp_rows_q_kernel<false>);
+            if (qbound)
+                return K >= 4 * 32 * QR_MAIN ? launch_q(lp_rows_q_kernel<true, true>) : launch_q(lp_rows_q_kernel<false, true>);
+            return K >= 4 * 32 * QR_MAIN ? launch_q(lp_rows_q_kernel<true, false>) : launch_q(lp_rows_q_kernel<false, false>);
         }
         auto launch =[&](auto kernel, int rpw) -> cudaError_t {
             const size_t smem = (size_t)ROW_WARPS * rpw * (sizeof(double) * KP_TILED + 4 * Q_PIECE);
@@ -1170,7 +1213,8 @@ cudaError_t launch_lp_rows(const double *models, int ld_models, CellRange cr, co
             if (e != cudaSuccess) return e;
             kernel<<<(unsigned)blocks, ROW_WARPS * 32, smem, st>>>(
                 models, ld_models, cr, row_off, row_cell_map, row_x, (const double4 *)row_const, row_snap, prep, K, sentinel,
-                table, ld_table, row_mode, which, zero_row, based, write_f64, zero_compact, qtable, q_row_bytes(K), row_range);
+                table, ld_table, row_mode, which, zero_row, based, write_f64, zero_compact, qtable, q_row_bytes(K), row_range,
+                qtable ? qbound : nullptr);
             return cudaGetLastError();
         };
         const bool norm = write_f64 != 0;  // rows that exist in fixed point only need no normalising constant
