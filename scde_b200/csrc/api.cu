@@ -397,18 +397,20 @@ int index_from_counts(scde_b200_ctx *ctx, LpTable &t, const int32_t *counts_dev,
     return SCDE_B200_OK;
 }
 
+// The device buffers of run_joint.  Joint j (W, Z, W8, zb): the j-th of the joints over the same cells that one run
+// computes together.  Side i (T, SR, S): the i-th side of a tcgen05 launch -- side 1 is the second joint, or the second
+// pass of a paired-pass launch.
 struct JointScratch {
-    DBuf<double> W, Z, zpart, T, spart;
-    DBuf<double> T2;    // T tiles of the second pass when two passes of randomizations share a launch
-    DBuf<int8_t> W8;
-    DBuf<uint32_t> SR;  // sentinel range of every (gene, boot) of one launch of the tcgen05 kernel
-    DBuf<uint32_t> SR2;
+    DBuf<double> W[2], Z[2], T[2];
+    DBuf<double> zpart, spart;  // base-sum and soft-max partial sums (every joint and side in turn, on one stream)
+    DBuf<int8_t> W8[2];
+    DBuf<uint32_t> SR[2];  // sentinel range of every (gene, boot) of one launch of the tcgen05 kernel
     DBuf<int32_t> lst_row, lst_cell, lst_len, order;
     DBuf<unsigned long long> total;  // running sums over the joints of one run: list lengths, then launch_prune_items' four
-    // pruning (launch_prune_items): Z extrema of the joint, bound sums of one launch (S2: the paired pass), live pieces and
-    // items of one launch, and the live count
-    DBuf<double> zb;
-    DBuf<int32_t> S, S2, items, n_live;
+    // pruning (launch_prune_items): Z extrema of each joint, bound sums of each side of one launch, live pieces and items
+    // of one launch, and the live count
+    DBuf<double> zb[2];
+    DBuf<int32_t> S[2], items, n_live;
     DBuf<uint8_t> live;
 };
 
@@ -419,7 +421,6 @@ struct DiffWorkspace {
     DBuf<int32_t> counts;  // [C][G] (column-major shard)
     LpTable table;
     JointScratch scr;
-    JointScratch scr2;  // the second of two joints computed in one launch (batch-corrected calls)
     DBuf<double> jp[4];
     DBuf<double> post, bpost, apost;  // [G][ld] gene-major ratio posteriors
     DBuf<double> tbuf;                // transposition scratch for downloads
@@ -433,22 +434,20 @@ struct DrawSets {
     const int32_t *gene_set = nullptr;
 };
 
-// A second joint over the SAME cells (and therefore the same entry lists) with its own draws, computed in the same
-// launches of the tcgen05 kernel: the two composition-sampled joints of a batch-corrected call (R/functions.R:355-357).
-struct TwinJoint {
-    const int32_t *boot_idx_dev;  // n_boot x D per draw set (the first joint's sets)
+// One joint of run_joint: its draws (n_boot x D per draw set, device) and its output
+struct Joint {
+    const int32_t *boot_idx_dev;
     int D;
     double *jp_dev;
-    JointScratch *scr;            // W, W8, Z, zpart, T, SR, spart of the second joint (the lists are the first joint's)
 };
 
-// The tcgen05 contraction of a joint whose operands run_joint has prepared, and of its twin (NULL: none) in the same
-// launches.  The launches raise bits in *status (read_status).
+// The tcgen05 contraction of joints[0 .. n_joints) (two: joints over the same cells and entry lists with their own draws)
+// whose operands run_joint has prepared.  The launches raise bits in *status (read_status).
 // prune (DESIGN.md 4.3): before each launch a bound pass and a decision find the (gene, piece) items the soft-max cannot
 // see; the contraction and the soft-max then skip them.  prune_stats (or NULL): launch_prune_items' four counters.
 int contract_joint_i8(scde_b200_ctx *ctx, const LpTable &t, const GeneLists &lists, JointScratch &scr, int n_w_rows,
-                      int n_boot, const DrawSets &sets, double scale, double *jp_dev, int ld_jp, int hot_rank,
-                      int32_t *status, const TwinJoint *twin, StageTimer *tm, bool prune, unsigned long long *prune_stats) {
+                      int n_boot, const DrawSets &sets, double scale, const Joint *joints, int n_joints, int ld_jp,
+                      int hot_rank, int32_t *status, StageTimer *tm, bool prune, unsigned long long *prune_stats) {
     cudaStream_t st = ctx->stream;
     const int passes = (n_boot + WP_TILED - 1) / WP_TILED;
     ContractI8Args q{};
@@ -456,18 +455,14 @@ int contract_joint_i8(scde_b200_ctx *ctx, const LpTable &t, const GeneLists &lis
     q.ldq = q_row_bytes(t.K);
     q.row_range = t.qrange.p;
     q.lists = lists;
-    q.W8 = scr.W8.p;
     q.n_w_rows = n_w_rows;
     q.n_boot = n_boot;
-    q.Z = scr.Z.p;
     q.gene_set = sets.gene_set;
     q.set_w8 = (int64_t)passes * n_w_rows * Q_WB;
     q.set_z = (int64_t)passes * WP_TILED * KP_TILED;
     q.scale = scale;
     q.sentinel = t.sentinel;
-    q.n_genes = t.n_genes;
     q.K = t.K;
-    q.jp = jp_dev;
     q.ld_jp = ld_jp;
     q.err = status;
     q.dbg = nullptr;
@@ -480,94 +475,70 @@ int contract_joint_i8(scde_b200_ctx *ctx, const LpTable &t, const GeneLists &lis
         SCDE_CUDA(cudaMemsetAsync(ctx->epi_dbg.p, 0, 3 * sizeof(unsigned long long), st));
         q.dbg = ctx->epi_dbg.p;
     }
-    SCDE_CUDA(scr.T.ensure(contract_tiled_scratch_doubles(t.n_genes)));
+    // More than 104 randomizations (R's default is 150) take several passes over the same lists and rows.  Two joints
+    // share every launch: (joint 0, pass ps) with (joint 1, pass ps).  One joint pairs its passes: ps with ps + 1, an odd
+    // last pass on its own.
+    const bool pass_pairs = n_joints == 1 && passes > 1 && ctx->opt.twin_batch_joints;
+    const int n_sides = (n_joints > 1 || pass_pairs) ? 2 : 1;
     const int max_genes = contract_tiled_max_genes();
-    SCDE_CUDA(scr.SR.ensure(contract_i8_range_words(t.n_genes < max_genes ? t.n_genes : max_genes)));
-    SCDE_CUDA(scr.spart.ensure(softmax_i8_scratch_doubles(t.n_genes < max_genes ? t.n_genes : max_genes)));
-    ContractI8Args q2 = q;  // the twin joint: same table, lists and schedule; its own W, Z, output
-    if (twin) {
-        JointScratch &s2 = *twin->scr;
-        SCDE_CUDA(s2.T.ensure(contract_tiled_scratch_doubles(t.n_genes)));
-        SCDE_CUDA(s2.SR.ensure(contract_i8_range_words(t.n_genes < max_genes ? t.n_genes : max_genes)));
-        SCDE_CUDA(s2.spart.ensure(softmax_i8_scratch_doubles(t.n_genes < max_genes ? t.n_genes : max_genes)));
-        q2.W8 = s2.W8.p;
-        q2.Z = s2.Z.p;
-        q2.jp = twin->jp_dev;
-        q.W8_twin = s2.W8.p;   // one launch of the contraction kernel computes both joints' T tiles
-        q.t_twin = s2.T.p;
+    const int mp = t.n_genes < max_genes ? t.n_genes : max_genes;
+    for (int i = 0; i < n_sides; ++i) {
+        SCDE_CUDA(scr.T[i].ensure(contract_tiled_scratch_doubles(t.n_genes)));
+        SCDE_CUDA(scr.SR[i].ensure(contract_i8_range_words(mp)));
+        if (prune) SCDE_CUDA(scr.S[i].ensure(prune_bound_ints(mp)));
     }
-    // More than 104 randomizations (R's default is 150): two passes over the same lists and rows.  Without a twin joint
-    // the passes are paired the same way -- pass ps and ps + 1 in one launch, on neighbouring SMs.
-    const bool pass_pairs = !twin && passes > 1 && ctx->opt.twin_batch_joints;
-    if (pass_pairs) {
-        SCDE_CUDA(scr.T2.ensure(contract_tiled_scratch_doubles(t.n_genes)));
-        SCDE_CUDA(scr.SR2.ensure(contract_i8_range_words(t.n_genes < max_genes ? t.n_genes : max_genes)));
-    }
+    SCDE_CUDA(scr.spart.ensure(softmax_i8_scratch_doubles(mp)));
     if (prune) {
-        const int mp = t.n_genes < max_genes ? t.n_genes : max_genes;
-        q.qbound = t.qb.p;
-        SCDE_CUDA(scr.zb.ensure(prune_zb_doubles(sets.n, n_boot)));
-        SCDE_CUDA(scr.S.ensure(prune_bound_ints(mp)));
-        if (pass_pairs) SCDE_CUDA(scr.S2.ensure(prune_bound_ints(mp)));
+        for (int j = 0; j < n_joints; ++j) SCDE_CUDA(scr.zb[j].ensure(prune_zb_doubles(sets.n, n_boot)));
         SCDE_CUDA(scr.live.ensure((size_t)mp));
         SCDE_CUDA(scr.items.ensure((size_t)mp * q_pieces(t.K)));
         SCDE_CUDA(scr.n_live.ensure(1));
-        const int e0 = tm ? tm->begin(st) : -1;
-        SCDE_CUDA(launch_z_bounds(q, sets.n, scr.zb.p, st));
-        if (twin) {
-            JointScratch &s2 = *twin->scr;
-            SCDE_CUDA(s2.zb.ensure(prune_zb_doubles(sets.n, n_boot)));
-            SCDE_CUDA(s2.S.ensure(prune_bound_ints(mp)));
-            SCDE_CUDA(launch_z_bounds(q2, sets.n, s2.zb.p, st));
-        }
-        if (tm) tm->end(SCDE_B200_T_BOUND, e0, st, twin ? 2 : 1);
+        q.qbound = t.qb.p;
+        q.items = scr.items.p;  // the contraction reads the live items launch_prune_items wrote
+        q.n_live = scr.n_live.p;
     }
+    auto side = [&](int j, int ps, int i) {  // joint j's pass ps as side i
+        return I8Side{scr.W8[j].p + (size_t)ps * n_w_rows * Q_WB, scr.Z[j].p + (size_t)ps * WP_TILED * KP_TILED, scr.T[i].p,
+                      scr.SR[i].p, scr.S[i].p, scr.zb[j].p, joints[j].jp_dev, ps};
+    };
+    struct Launch {
+        I8Side s[2];
+        int n;
+    };
+    std::vector<Launch> launches;
+    for (int ps = 0; ps < passes; ++ps) {
+        if (n_joints > 1)
+            launches.push_back({{side(0, ps, 0), side(1, ps, 1)}, 2});
+        else if (pass_pairs && ps + 1 < passes) {
+            launches.push_back({{side(0, ps, 0), side(0, ps + 1, 1)}, 2});
+            ++ps;
+        } else
+            launches.push_back({{side(0, ps, 0)}, 1});
+    }
+    if (prune) {
+        const int e0 = tm ? tm->begin(st) : -1;
+        for (int j = 0; j < n_joints; ++j) SCDE_CUDA(launch_z_bounds(q, scr.Z[j].p, sets.n, scr.zb[j].p, st));
+        if (tm) tm->end(SCDE_B200_T_BOUND, e0, st, n_joints);
+    }
+    const uint8_t *live = prune ? scr.live.p : nullptr;
     for (int g0 = 0; g0 < t.n_genes; g0 += max_genes) {
         const int n_pos = (t.n_genes - g0) < max_genes ? (t.n_genes - g0) : max_genes;
-        for (int ps = 0; ps < passes; ++ps) {
-            const bool pair = pass_pairs && ps + 1 < passes;
+        for (const Launch &l : launches) {
             int e0 = tm ? tm->begin(st) : -1;
-            SCDE_CUDA(launch_sentinel_ranges(q, g0, n_pos, ps, scr.SR.p, st));
-            if (twin) SCDE_CUDA(launch_sentinel_ranges(q2, g0, n_pos, ps, twin->scr->SR.p, st));
-            if (pair) SCDE_CUDA(launch_sentinel_ranges(q, g0, n_pos, ps + 1, scr.SR2.p, st));
-            if (tm) tm->end(SCDE_B200_T_OTHER, e0, st, (twin || pair) ? 2 : 1);
-            if (pair) {  // make_params adds the pass offset to both W pointers: the twin is the next pass
-                q.W8_twin = q.W8 + (size_t)n_w_rows * Q_WB;
-                q.t_twin = scr.T2.p;
-            }
+            for (int i = 0; i < l.n; ++i) SCDE_CUDA(launch_sentinel_ranges(q, g0, n_pos, l.s[i], st));
+            if (tm) tm->end(SCDE_B200_T_OTHER, e0, st, l.n);
             if (prune) {
                 e0 = tm ? tm->begin(st) : -1;
-                int32_t *S_twin = twin ? twin->scr->S.p : pair ? scr.S2.p : nullptr;
-                SCDE_CUDA(launch_bound_pass(q, g0, n_pos, ps, ctx->n_sm, scr.S.p, S_twin, st));
-                const PruneSide s0{scr.SR.p, scr.S.p, scr.zb.p, ps};
-                const PruneSide s1 = twin ? PruneSide{twin->scr->SR.p, S_twin, twin->scr->zb.p, ps}
-                                          : PruneSide{scr.SR2.p, S_twin, scr.zb.p, ps + 1};
-                SCDE_CUDA(launch_prune_items(q, g0, n_pos, s0, (twin || pair) ? &s1 : nullptr, scr.live.p, scr.items.p,
-                                             scr.n_live.p, prune_stats, st));
+                SCDE_CUDA(launch_bound_pass(q, g0, n_pos, l.s, l.n, ctx->n_sm, st));
+                SCDE_CUDA(launch_prune_items(q, g0, n_pos, l.s, l.n, scr.live.p, scr.items.p, scr.n_live.p, prune_stats, st));
                 if (tm) tm->end(SCDE_B200_T_BOUND, e0, st, 3);
-                q.items = scr.items.p;
-                q.n_live = scr.n_live.p;
             }
             e0 = tm ? tm->begin(st) : -1;
-            SCDE_CUDA(launch_contract_i8_pass(q, g0, n_pos, ps, ctx->n_sm, scr.T.p, st));
-            q.items = nullptr;
-            q.n_live = nullptr;
-            if (pair) {
-                q.W8_twin = nullptr;
-                q.t_twin = nullptr;
-            }
-            const uint8_t *live = prune ? scr.live.p : nullptr;
+            SCDE_CUDA(launch_contract_i8_pass(q, g0, n_pos, l.s, l.n, ctx->n_sm, st));
             if (tm) tm->end(SCDE_B200_T_CONTRACT, e0, st, 1);
             e0 = tm ? tm->begin(st) : -1;
-            SCDE_CUDA(launch_softmax_i8(q, g0, n_pos, ps, scr.T.p, scr.SR.p, scr.spart.p, ctx->n_sm, st, live));
-            if (twin)
-                SCDE_CUDA(launch_softmax_i8(q2, g0, n_pos, ps, twin->scr->T.p, twin->scr->SR.p, twin->scr->spart.p,
-                                            ctx->n_sm, st, live));
-            if (pair) {
-                SCDE_CUDA(launch_softmax_i8(q, g0, n_pos, ps + 1, scr.T2.p, scr.SR2.p, scr.spart.p, ctx->n_sm, st, live));
-                ++ps;
-            }
-            if (tm) tm->end(SCDE_B200_T_SOFTMAX, e0, st, (twin || pair) ? 4 : 2);
+            for (int i = 0; i < l.n; ++i) SCDE_CUDA(launch_softmax_i8(q, g0, n_pos, l.s[i], scr.spart.p, ctx->n_sm, st, live));
+            if (tm) tm->end(SCDE_B200_T_SOFTMAX, e0, st, 2 * l.n);
         }
     }
     if (q.dbg) {
@@ -594,7 +565,7 @@ int contract_joint_fp64(scde_b200_ctx *ctx, Contraction kernel, const LpTable &t
     a.table = t.table.p;
     a.ld_table = t.ld;
     a.lists = lists;
-    a.W = scr.W.p;
+    a.W = scr.W[0].p;
     a.n_w_rows = n_w_rows;
     a.n_boot = n_boot;
     a.Z = Z;
@@ -616,8 +587,8 @@ int contract_joint_fp64(scde_b200_ctx *ctx, Contraction kernel, const LpTable &t
     const int e0 = tm ? tm->begin(st) : -1;
     int nl = 0;
     if (tiled) {
-        SCDE_CUDA(scr.T.ensure(contract_tiled_scratch_doubles(t.n_genes)));
-        SCDE_CUDA(launch_contract_tiled(a, ctx->n_sm, scr.T.p, st, &nl));
+        SCDE_CUDA(scr.T[0].ensure(contract_tiled_scratch_doubles(t.n_genes)));
+        SCDE_CUDA(launch_contract_tiled(a, ctx->n_sm, scr.T[0].p, st, &nl));
     }
     else
         SCDE_CUDA(launch_contract_generic(a, st, &nl));
@@ -625,81 +596,74 @@ int contract_joint_fp64(scde_b200_ctx *ctx, Contraction kernel, const LpTable &t
     return SCDE_B200_OK;
 }
 
-// jp_dev[G][ld_jp] = joint posterior of the listed cells under the draws boot_idx_dev (n_boot x D per draw set, device), on
-// the contraction kernel k selects.  The tcgen05 launches raise bits in the device word *status, which the caller has zeroed
-// (the second joint of a twin pair that did not share the launches adds to the first one's word).
-// twin (optional): see TwinJoint; only honoured on the tcgen05 path (the caller checks the return flag *twin_done and runs
-// the second joint on its own otherwise).
+// joints[j].jp_dev[G][ld_jp] = joint posterior of the listed cells under joint j's draws, for n_joints (1 or 2) joints over
+// the same cells, on the contraction kernel k selects.  Two joints share the entry lists and the launches of the tcgen05
+// kernel when both can run on it and twin_batch_joints is on; otherwise they run one after the other.  The tcgen05
+// launches raise bits in the device word *status, which the caller has zeroed and both joints share.
 int run_joint(scde_b200_ctx *ctx, ContractChoice k, const LpTable &t, const int32_t *cell_ids_dev, int n_list,
-              const int32_t *boot_idx_dev, int n_boot, int D, const DrawSets &sets, double scale, double *jp_dev,
-              int ld_jp, JointScratch &scr, int32_t *status, StageTimer *tm, bool count_entries,
-              const TwinJoint *twin = nullptr, bool *twin_done = nullptr) {
+              const Joint *joints, int n_joints, int n_boot, const DrawSets &sets, double scale, int ld_jp,
+              JointScratch &scr, int32_t *status, StageTimer *tm, bool count_entries) {
     cudaStream_t st = ctx->stream;
     const int n_w_rows = round_up(n_list + 1, 16);  // at least one all-zero row after the cells (list padding)
     const int passes = (n_boot + WP_TILED - 1) / WP_TILED;
     const int ld_lst = round_up(n_list, 32);
+    const bool zb = t.zero_base && t.ld <= KP_TILED;
+    auto i8_for = [&](const Joint &jt) {
+        return zb && t.has_q && k.kernel == Contraction::I8 && contract_i8_supported(t.K, t.ld, ld_lst, jt.D);
+    };
+    if (n_joints > 1 && !(i8_for(joints[0]) && i8_for(joints[1]) && ctx->opt.twin_batch_joints)) {
+        for (int j = 0; j < n_joints; ++j)
+            TRY(run_joint(ctx, k, t, cell_ids_dev, n_list, joints + j, 1, n_boot, sets, scale, ld_jp, scr, status, tm,
+                          count_entries));
+        return SCDE_B200_OK;
+    }
+    const bool i8 = i8_for(joints[0]);
+    if (k.forced && !i8) {
+        set_error("tcgen05 int8 contraction forced but unsupported here (K=%d, zero-base form %d)", t.K, (int)zb);
+        return SCDE_B200_EINVAL;
+    }
     const int S = sets.n;
     const size_t w_set = (size_t)passes * n_w_rows * WS_TILED, z_set = (size_t)passes * WP_TILED * t.ld;
-    const size_t w8_set = (size_t)passes * n_w_rows * Q_WB, draws_set = (size_t)n_boot * D;
-    SCDE_CUDA(scr.W.ensure(S * w_set));
+    const size_t w8_set = (size_t)passes * n_w_rows * Q_WB;
     SCDE_CUDA(scr.lst_row.ensure((size_t)t.n_genes * ld_lst));
     SCDE_CUDA(scr.lst_cell.ensure((size_t)t.n_genes * ld_lst));
     SCDE_CUDA(scr.lst_len.ensure((size_t)t.n_genes));
     SCDE_CUDA(scr.order.ensure((size_t)t.n_genes));
     SCDE_CUDA(scr.total.ensure(5));
-    const bool zb = t.zero_base && t.ld <= KP_TILED;
-    if (zb) {
-        SCDE_CUDA(scr.Z.ensure(S * z_set));
-        SCDE_CUDA(scr.zpart.ensure(base_sum_scratch_doubles(n_boot, t.ld)));
+    if (zb) SCDE_CUDA(scr.zpart.ensure(base_sum_scratch_doubles(n_boot, t.ld)));
+    for (int j = 0; j < n_joints; ++j) {
+        SCDE_CUDA(scr.W[j].ensure(S * w_set));
+        if (zb) SCDE_CUDA(scr.Z[j].ensure(S * z_set));
+        if (i8) SCDE_CUDA(scr.W8[j].ensure(S * w8_set));
     }
     const int e0 = tm ? tm->begin(st) : -1;
-    for (int s = 0; s < S; ++s)
-        SCDE_CUDA(launch_build_w(boot_idx_dev + s * draws_set, n_boot, D, n_list, scr.W.p + s * w_set, n_w_rows, st));
-    SCDE_CUDA(cudaMemsetAsync(jp_dev, 0, sizeof(double) * (size_t)t.n_genes * ld_jp, st));
     GeneLists lists{scr.lst_row.p, scr.lst_cell.p, scr.lst_len.p, scr.order.p, ld_lst};
-    const bool i8 = zb && t.has_q && k.kernel == Contraction::I8 && contract_i8_supported(t.K, t.ld, ld_lst, D);
-    const bool tw = twin && i8 && contract_i8_supported(t.K, t.ld, ld_lst, twin->D) && ctx->opt.twin_batch_joints;
-    if (twin_done) *twin_done = tw;
-    if (k.forced && !i8) {
-        set_error("tcgen05 int8 contraction forced but unsupported here (K=%d, zero-base form %d)", t.K, (int)zb);
-        return SCDE_B200_EINVAL;
-    }
     const int hot_rank = i8 ? ctx->opt.hot_rank : -1;  // only the tcgen05 kernel's producers know the hot bit
     SCDE_CUDA(launch_build_lists(t.ridx.p, t.ld_ridx, cell_ids_dev, n_list, t.n_genes, zb ? t.zero_row.p : nullptr,
                                  zb ? t.based.p : nullptr, 0, lists, count_entries ? scr.total.p : nullptr, st, hot_rank,
-                                 tw ? 2 : 1));
-    if (zb)
+                                 n_joints));
+    for (int j = 0; j < n_joints; ++j) {  // each joint's W, base sums and W8, and its output zeroed
+        const Joint &jt = joints[j];
+        const size_t draws_set = (size_t)n_boot * jt.D;
         for (int s = 0; s < S; ++s)
-            SCDE_CUDA(launch_base_sum(t.table.p, t.ld, t.zero_row.p, t.based.p, cell_ids_dev, n_list, scr.W.p + s * w_set,
-                                      n_w_rows, n_boot, scr.Z.p + s * z_set, scr.zpart.p, st, t.zero_compact));
-    // W8 of all sets in one conversion: the sets' blocks are consecutive rows
-    if (tw) {  // the second joint's W, base sums and output
-        JointScratch &s2 = *twin->scr;
-        const size_t twin_draws_set = (size_t)n_boot * twin->D;
-        SCDE_CUDA(s2.W.ensure(S * w_set));
-        SCDE_CUDA(s2.Z.ensure(S * z_set));
-        SCDE_CUDA(s2.zpart.ensure(base_sum_scratch_doubles(n_boot, t.ld)));
-        SCDE_CUDA(s2.W8.ensure(S * w8_set));
-        for (int s = 0; s < S; ++s)
-            SCDE_CUDA(launch_build_w(twin->boot_idx_dev + s * twin_draws_set, n_boot, twin->D, n_list, s2.W.p + s * w_set,
-                                     n_w_rows, st));
-        SCDE_CUDA(cudaMemsetAsync(twin->jp_dev, 0, sizeof(double) * (size_t)t.n_genes * ld_jp, st));
-        for (int s = 0; s < S; ++s)
-            SCDE_CUDA(launch_base_sum(t.table.p, t.ld, t.zero_row.p, t.based.p, cell_ids_dev, n_list, s2.W.p + s * w_set,
-                                      n_w_rows, n_boot, s2.Z.p + s * z_set, s2.zpart.p, st, t.zero_compact));
-        SCDE_CUDA(launch_w_to_i8(s2.W.p, S * n_w_rows, n_boot, s2.W8.p, status, st));
-    }
-    if (i8) {
-        SCDE_CUDA(scr.W8.ensure(S * w8_set));
-        SCDE_CUDA(launch_w_to_i8(scr.W.p, S * n_w_rows, n_boot, scr.W8.p, status, st));
+            SCDE_CUDA(launch_build_w(jt.boot_idx_dev + s * draws_set, n_boot, jt.D, n_list, scr.W[j].p + s * w_set, n_w_rows,
+                                     st));
+        SCDE_CUDA(cudaMemsetAsync(jt.jp_dev, 0, sizeof(double) * (size_t)t.n_genes * ld_jp, st));
+        if (zb)
+            for (int s = 0; s < S; ++s)
+                SCDE_CUDA(launch_base_sum(t.table.p, t.ld, t.zero_row.p, t.based.p, cell_ids_dev, n_list,
+                                          scr.W[j].p + s * w_set, n_w_rows, n_boot, scr.Z[j].p + s * z_set, scr.zpart.p, st,
+                                          t.zero_compact));
+        // W8 of all sets in one conversion: the sets' blocks are consecutive rows
+        if (i8) SCDE_CUDA(launch_w_to_i8(scr.W[j].p, S * n_w_rows, n_boot, scr.W8[j].p, status, st));
     }
     // build_w is a memset and a kernel, base_sum two kernels: per extra set
-    if (tm) tm->end(SCDE_B200_T_OTHER, e0, st, (zb ? 5 : 3) + (i8 ? 1 : 0) + (tw ? 5 : 0) + (S - 1) * ((zb ? 4 : 2) + (tw ? 4 : 0)));
+    if (tm) tm->end(SCDE_B200_T_OTHER, e0, st, n_joints * ((zb ? 5 : 3) + (S - 1) * (zb ? 4 : 2)) + (i8 ? 1 : 0));
     if (!i8)
-        return contract_joint_fp64(ctx, k.kernel, t, lists, scr, zb ? scr.Z.p : nullptr, n_w_rows, n_boot, sets, scale,
-                                   jp_dev, ld_jp, tm);
-    return contract_joint_i8(ctx, t, lists, scr, n_w_rows, n_boot, sets, scale, jp_dev, ld_jp, hot_rank, status,
-                             tw ? twin : nullptr, tm, t.has_bounds && ctx->opt.prune_pieces && n_list >= PRUNE_MIN_CELLS,
+        return contract_joint_fp64(ctx, k.kernel, t, lists, scr, zb ? scr.Z[0].p : nullptr, n_w_rows, n_boot, sets, scale,
+                                   joints[0].jp_dev, ld_jp, tm);
+    return contract_joint_i8(ctx, t, lists, scr, n_w_rows, n_boot, sets, scale, joints, n_joints, ld_jp, hot_rank, status, tm,
+                             t.has_bounds && ctx->opt.prune_pieces && n_list >= PRUNE_MIN_CELLS,
                              count_entries ? scr.total.p + 1 : nullptr);
 }
 
@@ -1468,7 +1432,8 @@ static int log_boot_impl(scde_b200_ctx *ctx, const double *models, int32_t n_cel
         }
         TRY(validate_index(boot_idx, (size_t)nb * dd, 0, n_cells, "boot_idx"));
         TRY(upload(d_boot, boot_idx, (size_t)nb * dd, st));
-        TRY(run_joint(ctx, k, t, nullptr, n_cells, d_boot.p, nb, dd, {}, scale, d_jp.p, ld_jp, scr, status.p, nullptr, false));
+        const Joint jt{d_boot.p, dd, d_jp.p};
+        TRY(run_joint(ctx, k, t, nullptr, n_cells, &jt, 1, nb, {}, scale, ld_jp, scr, status.p, nullptr, false));
     }
     SCDE_CUDA(d_out.ensure((size_t)n_genes * n_grid));
     SCDE_CUDA(launch_transpose_out(d_jp.p, ld_jp, n_genes, n_grid, d_out.p, st));
@@ -1605,8 +1570,9 @@ static int jpmat_common(scde_b200_ctx *ctx, const double *matl, int n_mat, int n
     JointScratch scr;
     if (n_boot > 0) {
         // not divided by n_boot: src/jpmatLogBoot.cpp:36-38 (no fixed-point table: no tcgen05 launch, no status word)
-        TRY(run_joint(ctx, contraction_choice(ctx), t, nullptr, n_mat, d_boot.p, n_boot, D, {}, 1.0, d_jp.p, t.ld, scr, nullptr,
-                      nullptr, false));
+        const Joint jt{d_boot.p, D, d_jp.p};
+        TRY(run_joint(ctx, contraction_choice(ctx), t, nullptr, n_mat, &jt, 1, n_boot, {}, 1.0, t.ld, scr, nullptr, nullptr,
+                      false));
     } else {
         SCDE_CUDA(cudaMemsetAsync(d_jp.p, 0, sizeof(double) * (size_t)n_rows * t.ld, st));
     }
@@ -1965,22 +1931,19 @@ int scde_b200_probe_prune_i8(scde_b200_ctx *ctx, const int8_t *qtable, int32_t n
     q.ldq = ldq;
     q.row_range = row_range ? d_rr.p : nullptr;
     q.lists = GeneLists{d_row.p, d_cell.p, d_len.p, nullptr, ld_lst};
-    q.W8 = d_w.p;
     q.n_w_rows = n_w_rows;
     q.n_boot = WP_TILED;
-    q.Z = nullptr;
     q.scale = 1.0;
     q.sentinel = -1.0e300;
-    q.n_genes = n_genes;
     q.K = n_grid;
-    q.jp = nullptr;
     q.ld_jp = 0;
     q.err = status.p;
     q.item_order = ctx->opt.item_order;
     q.hot_rank = -1;
     q.cold_evict_first = 0;
     q.ring_stages = ctx->opt.ring_stages;
-    SCDE_CUDA(launch_sentinel_ranges(q, 0, n_genes, 0, d_sr.p, st));
+    I8Side side{d_w.p, nullptr, d_t.p, d_sr.p, nullptr, nullptr, nullptr, 0};
+    SCDE_CUDA(launch_sentinel_ranges(q, 0, n_genes, side, st));
     DBuf<int8_t> d_qb;
     DBuf<double> d_z, d_zb, d_lb, d_ub;
     DBuf<int32_t> d_s, d_items, d_nlive;
@@ -1989,7 +1952,6 @@ int scde_b200_probe_prune_i8(scde_b200_ctx *ctx, const int8_t *qtable, int32_t n
         TRY(upload(d_qb, qbound, (size_t)n_rows * Q_BW, st));
         if (z) TRY(upload(d_z, z, (size_t)WP_TILED * KP_TILED, st));
         q.qbound = d_qb.p;
-        q.Z = z ? d_z.p : nullptr;
         SCDE_CUDA(d_zb.ensure(prune_zb_doubles(1, WP_TILED)));
         SCDE_CUDA(d_s.ensure(prune_bound_ints(n_genes)));
         SCDE_CUDA(d_lb.ensure((size_t)n_genes * WP_TILED));
@@ -1997,14 +1959,14 @@ int scde_b200_probe_prune_i8(scde_b200_ctx *ctx, const int8_t *qtable, int32_t n
         SCDE_CUDA(d_live.ensure((size_t)n_genes));
         SCDE_CUDA(d_items.ensure((size_t)n_genes * q_pieces(n_grid)));
         SCDE_CUDA(d_nlive.ensure(1));
-        SCDE_CUDA(launch_z_bounds(q, 1, d_zb.p, st));
-        SCDE_CUDA(launch_bound_pass(q, 0, n_genes, 0, ctx->n_sm, d_s.p, nullptr, st));
-        SCDE_CUDA(launch_prune_items(q, 0, n_genes, PruneSide{d_sr.p, d_s.p, d_zb.p, 0}, nullptr, d_live.p, d_items.p,
-                                     d_nlive.p, nullptr, st, d_lb.p, d_ub.p));
-        q.Z = nullptr;
+        side.S = d_s.p;
+        side.zb = d_zb.p;
+        SCDE_CUDA(launch_z_bounds(q, z ? d_z.p : nullptr, 1, d_zb.p, st));
+        SCDE_CUDA(launch_bound_pass(q, 0, n_genes, &side, 1, ctx->n_sm, st));
+        SCDE_CUDA(launch_prune_items(q, 0, n_genes, &side, 1, d_live.p, d_items.p, d_nlive.p, nullptr, st, d_lb.p, d_ub.p));
     }
-    SCDE_CUDA(launch_contract_i8_pass(q, 0, n_genes, 0, ctx->n_sm, d_t.p, st));
-    SCDE_CUDA(launch_finalize_t(q, n_genes, d_t.p, d_sr.p, st));
+    SCDE_CUDA(launch_contract_i8_pass(q, 0, n_genes, &side, 1, ctx->n_sm, st));
+    SCDE_CUDA(launch_finalize_t(q, n_genes, side, st));
     SCDE_CUDA(cudaMemcpyAsync(t_out, d_t.p, sizeof(double) * nt, cudaMemcpyDeviceToHost, st));
     if (qbound) {
         SCDE_CUDA(cudaMemcpyAsync(lb_out, d_lb.p, sizeof(double) * n_genes * WP_TILED, cudaMemcpyDeviceToHost, st));
@@ -2533,8 +2495,9 @@ static int diff_run_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, bool chunked
     bool front_done = false, joint0_done = false;
     const DrawSets sets{j->chunks.n_sets(), j->gene_set.p};
     auto group_joint = [&](int i) {  // cells of one factor level, draws are local indices (R/functions.R:372-374)
-        return run_joint(ctx, k, j->ws->table, j->cell_ids[i].p, j->n_group[i], j->boot_ptr[i], j->n_boot, j->D[i], sets,
-                         (double)j->n_boot, j->ws->jp[i].p, ld, j->ws->scr, j->status.p + i, &tm, true);
+        const Joint jt{j->boot_ptr[i], j->D[i], j->ws->jp[i].p};
+        return run_joint(ctx, k, j->ws->table, j->cell_ids[i].p, j->n_group[i], &jt, 1, j->n_boot, sets, (double)j->n_boot,
+                         ld, j->ws->scr, j->status.p + i, &tm, true);
     };
     if (chunked_counts) {
         TRY(front_chunked(ctx, j, 0, &front_done));
@@ -2573,13 +2536,9 @@ static int diff_run_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, bool chunked
         if (j->bmodels.m.p) TRY(fill_rows(ctx, j->ws->table, j->bmodels, j->mag.p, &tm));
         // the two composition-sampled joints walk the same cells and rows with different draws: one launch of the contraction
         // kernel for both, items paired on neighbouring SMs, so the table is pulled from DRAM once for the two
-        TwinJoint tw{j->boot_ptr[3], j->D[3], j->ws->jp[3].p, &j->ws->scr2};
-        bool twin_done = false;
-        TRY(run_joint(ctx, k, j->ws->table, nullptr, C, j->boot_ptr[2], j->n_boot, j->D[2], sets, (double)j->n_boot,
-                      j->ws->jp[2].p, ld, j->ws->scr, j->status.p + 2, &tm, true, &tw, &twin_done));
-        if (!twin_done)
-            TRY(run_joint(ctx, k, j->ws->table, nullptr, C, j->boot_ptr[3], j->n_boot, j->D[3], sets, (double)j->n_boot,
-                          j->ws->jp[3].p, ld, j->ws->scr, j->status.p + 2, &tm, true));
+        const Joint batch[2] = {{j->boot_ptr[2], j->D[2], j->ws->jp[2].p}, {j->boot_ptr[3], j->D[3], j->ws->jp[3].p}};
+        TRY(run_joint(ctx, k, j->ws->table, nullptr, C, batch, 2, j->n_boot, sets, (double)j->n_boot, ld, j->ws->scr,
+                      j->status.p + 2, &tm, true));
     }
     const int e0 = tm.begin(st);
     RatioPasses r = ratio_passes(G, K, ld, j->prior_y.p, j->zi.p, j->zi_adj.p, j->n_zero);
@@ -2971,27 +2930,22 @@ int shard_contrasts(DatasetShard &sh, const ContrastPlan &p, const scde_b200_con
     auto batch_draws = [&](int b) { return sh.bdraws.p + sh_bdraw_off[b]; };
     auto group_joint = [&](int s, ContractChoice kk, bool count) {
         const int n = (int)(p.cell_off[s + 1] - p.cell_off[s]);
-        return run_joint(ctx, kk, t, sh.cells.p + p.cell_off[s], n, group_draws(s), p.n_boot, n, sets, (double)p.n_boot,
-                         sh.bank.p + s * slot_sz, ld, ws->scr, sh.jflags.p + s, &tm, count);
+        const Joint jt{group_draws(s), n, sh.bank.p + s * slot_sz};
+        return run_joint(ctx, kk, t, sh.cells.p + p.cell_off[s], n, &jt, 1, p.n_boot, sets, (double)p.n_boot, ld, ws->scr,
+                         sh.jflags.p + s, &tm, count);
     };
-    auto batch_joint = [&](int b, ContractChoice kk, bool count, const TwinJoint *tw, bool *twin_done) {
-        return run_joint(ctx, kk, t, nullptr, sh.C, batch_draws(b), p.n_boot, p.bslot_D[b], sets, (double)p.n_boot,
-                         sh.bbank.p + b * slot_sz, ld, ws->scr, sh.jflags.p + n_slots + b / 2, &tm, count, tw, twin_done);
+    // batch joints b .. b + n - 1 (n <= 2); a pair of joints shares status word n_slots + b / 2
+    auto batch_joints = [&](int b, int n, ContractChoice kk, bool count) {
+        auto joint = [&](int i) { return Joint{batch_draws(i), p.bslot_D[i], sh.bbank.p + i * slot_sz}; };
+        const Joint js[2] = {joint(b), joint(b + n - 1)};
+        return run_joint(ctx, kk, t, nullptr, sh.C, js, n, p.n_boot, sets, (double)p.n_boot, ld, ws->scr,
+                         sh.jflags.p + n_slots + b / 2, &tm, count);
     };
     for (int s = 0; s < n_slots; ++s) TRY(group_joint(s, k, true));
     if (p.has_batch) {
         if (p.batch_models) TRY(ensure_rows(sh, 1, k, &tm));
         // distinct compositions in pairs: one launch of the tcgen05 kernel for two joints over the same cells and rows
-        for (int b = 0; b < n_bslots; b += 2) {
-            bool twin_done = false;
-            if (b + 1 < n_bslots) {
-                TwinJoint tw{batch_draws(b + 1), p.bslot_D[b + 1], sh.bbank.p + (b + 1) * slot_sz, &ws->scr2};
-                TRY(batch_joint(b, k, true, &tw, &twin_done));
-                if (!twin_done) TRY(batch_joint(b + 1, k, true, nullptr, nullptr));
-            } else {
-                TRY(batch_joint(b, k, true, nullptr, nullptr));
-            }
-        }
+        for (int b = 0; b < n_bslots; b += 2) TRY(batch_joints(b, n_bslots - b < 2 ? 1 : 2, k, true));
     }
     SCDE_CUDA(cudaStreamSynchronize(st));
     std::vector<int32_t> flags(n_words);
@@ -3010,7 +2964,7 @@ int shard_contrasts(DatasetShard &sh, const ContrastPlan &p, const scde_b200_con
             if (flags[n_slots + b / 2] & (1 | 4)) {
                 if (!rows) TRY(ensure_rows(sh, p.batch_models ? 1 : 0, {Contraction::Tiled}, &tm));
                 rows = true;
-                TRY(batch_joint(b, {Contraction::Tiled}, false, nullptr, nullptr));
+                TRY(batch_joints(b, 1, {Contraction::Tiled}, false));
             }
     }
     // ratio and summary: every contrast in one launch per pass; the 2K-1 posteriors that feed the adjusted pass (or that

@@ -233,29 +233,24 @@ cudaError_t launch_quantize_rows(const double *table, int ld_table, int K, int64
                                  uint32_t *row_range, int8_t *qbound, cudaStream_t st);
 // W8[pass][row][128] = (int8) W[pass][row][0..104); *flag |= 1 if a multiplicity exceeds 127
 cudaError_t launch_w_to_i8(const double *W, int n_w_rows, int n_boot, int8_t *W8, int32_t *flag, cudaStream_t st);
+// What the sides of a launch share (see I8Side)
 struct ContractI8Args {
     const int8_t *qtable;
     int ldq;
     const uint32_t *row_range;  // [rows] klo | khi << 16 (NULL: no row holds a sentinel)
     GeneLists lists;   // ld a multiple of 32, lists padded to a multiple of 32 with zero-W entries
-    const int8_t *W8;  // pass-major [ceil(n_boot/104)][n_w_rows][128]
     int n_w_rows;
-    int n_boot;
-    const double *Z;   // [ceil(n_boot/104)*104][416] or NULL
+    int n_boot;        // boots of every side's joint
     // Draw sets: gene_set[gene] (NULL: one set) selects the W8 and Z of the gene's set, gene_set[gene] * set_w8 bytes and
-    // gene_set[gene] * set_z doubles after the first set's (W8 [set][pass][n_w_rows][128]; the twin's W8 likewise)
+    // gene_set[gene] * set_z doubles after the first set's (W8 [set][pass][n_w_rows][128], Z [set][pass * 104 + b][416])
     const int32_t *gene_set;
     int64_t set_w8, set_z;
     double scale;
     double sentinel;   // the "log 0" value of the FP64 table
-    int n_genes, K;
-    double *jp;
+    int K;
     int ld_jp;
     int32_t *err;      // device flag, |= 2 if the kernel's watchdog fired, |= 4 if the sentinel ranges need the FP64 kernel
     unsigned long long *dbg;  // optional [3] cycle counters of the epilogue (see contract_i8.cu), or NULL
-    const int8_t *W8_twin;  // twin launch (launch_contract_i8_pass only): a second joint over the SAME cells and lists with its
-    double *t_twin;         // own draws -- its W (layout as W8) and its T scratch; NULL = one joint.  The sentinel ranges
-                            // and the soft-max of the second joint are separate launches with W8 = W8_twin.
     int item_order;    // 0: item = (gene, piece), a gene's pieces on neighbouring SMs; 1: piece-major (all SMs walk the same
                        // 512-byte piece of the rows at the same time, so rows shared between genes are L2 hits more often)
     int hot_rank;      // >= 0: list entries carry bit 30 of `cell` when the row's rank within its cell is <= hot_rank; such
@@ -266,52 +261,61 @@ struct ContractI8Args {
     const int32_t *items;  // launch_contract_i8_pass: contract only the live items, items[0 .. *n_live) (launch_prune_items);
     const int32_t *n_live; // NULL = every item
 };
+// One side of a launch: the boots of one joint in one pass.  A launch of the contraction (and of the bound pass) computes
+// one side or two over the same genes and lists; with two, items come in pairs on neighbouring SMs, so the second gather
+// of a table row is an L2 hit.  The two sides are two joints over the same cells (their passes alike), or passes ps and
+// ps + 1 of one joint.  The sentinel ranges, the soft-max and the Z extrema are launched per side or per joint.
+struct I8Side {
+    const int8_t *W8;   // the pass's W rows [n_w_rows][128] of the first draw set
+    const double *Z;    // the pass's base sums [104][416] of the first draw set, or NULL
+    double *T;          // T tiles [n_pos][104][416] of one launch
+    uint32_t *SR;       // sentinel ranges [n_pos][128] of one launch
+    int32_t *S;         // bound sums [n_pos][104][Q_BW] of one launch (pruning)
+    const double *zb;   // the joint's Z extrema (launch_z_bounds; pruning)
+    double *jp;         // the joint's output [n_genes][ld_jp]
+    int pass;
+};
 constexpr int32_t LIST_HOT_BIT = 1 << 30;  // in GeneLists::cell (W row ids are < 65536)
 // n_draws: draws per randomization (the plane sums are combined pairwise in 32 bits: 257 * 128 * draws < 2^31)
 bool contract_i8_supported(int K, int ld_table, int ld_lst, int n_draws);
 size_t contract_i8_range_words(int n_genes);  // uint32 words of the (gene, boot) sentinel-range scratch
-// sr_scratch[n_pos][128] = sentinel range of every (gene, boot) of genes order[g0 .. g0 + n_pos), boots of `pass`
+// s.SR[n_pos][128] = sentinel range of every (gene, boot) of genes order[g0 .. g0 + n_pos), boots of the side
 // (no-op when a.row_range == NULL)
-cudaError_t launch_sentinel_ranges(const ContractI8Args &a, int g0, int n_pos, int pass, uint32_t *sr_scratch,
-                                   cudaStream_t st);
-// one launch: genes order[g0 .. g0 + n_pos) (n_pos <= contract_tiled_max_genes()), boots [104 pass, 104 pass + 104);
-// writes 2^29 * T[boot, grid] as exact 64-bit integers (without the zero-count base, without sentinels) into t_scratch
-// ([n_pos][104][416], contract_tiled_scratch_doubles()) -- follow with launch_softmax_i8
-cudaError_t launch_contract_i8_pass(const ContractI8Args &a, int g0, int n_pos, int pass, int n_sm, double *t_scratch,
+cudaError_t launch_sentinel_ranges(const ContractI8Args &a, int g0, int n_pos, const I8Side &s, cudaStream_t st);
+// one launch over the sides s[0 .. n_sides) (1 or 2): genes order[g0 .. g0 + n_pos) (n_pos <= contract_tiled_max_genes()),
+// boots [104 pass, 104 pass + 104) of each side's joint; writes 2^29 * T[boot, grid] as exact 64-bit integers (without the
+// zero-count base, without sentinels) into each side's T ([n_pos][104][416], contract_tiled_scratch_doubles()) -- follow
+// with launch_softmax_i8.  The kernel stores the boots of side 0's pass: a second side with fewer (a ragged last pass)
+// relies on its W rows being zero beyond its boots.
+cudaError_t launch_contract_i8_pass(const ContractI8Args &a, int g0, int n_pos, const I8Side *s, int n_sides, int n_sm,
                                     cudaStream_t st);
-// the rest of the gene: a.jp[gene][k] (+)= sum_b softmax_k(2^-29 T + Z)[k] / a.scale with the sentinel ranges `sr` (what
+// the rest of the gene: s.jp[gene][k] (+)= sum_b softmax_k(2^-29 T + Z)[k] / a.scale with the sentinel ranges s.SR (what
 // launch_sentinel_ranges wrote; required when a.row_range != NULL); part_scratch: softmax_i8_scratch_doubles(n_pos)
 size_t softmax_i8_scratch_doubles(int n_pos);
 // live (NULL: every piece): the pieces launch_prune_items left live, whose T tiles are the only ones written
-cudaError_t launch_softmax_i8(const ContractI8Args &a, int g0, int n_pos, int pass, const double *t_scratch, const uint32_t *sr,
-                              double *part_scratch, int n_sm, cudaStream_t st, const uint8_t *live = nullptr);
+cudaError_t launch_softmax_i8(const ContractI8Args &a, int g0, int n_pos, const I8Side &s, double *part_scratch, int n_sm,
+                              cudaStream_t st, const uint8_t *live = nullptr);
 // ---- pruning (DESIGN.md 4.3): (gene, piece) items whose grid points the soft-max cannot see are not contracted
-// zb: prune_zb_doubles() doubles, the Z extrema of every (set, pass, boot) of the joint (a.Z, a.n_boot, a.K), once per joint
+// zb: prune_zb_doubles() doubles, the Z extrema of every (set, pass, boot) of a joint (its Z, a.n_boot, a.K), once per joint
 size_t prune_zb_doubles(int n_sets, int n_boot);
-cudaError_t launch_z_bounds(const ContractI8Args &a, int n_sets, double *zb, cudaStream_t st);
-// S[n_pos][104][Q_BW] = the sums of the drawn rows' bound rows (a.qbound) of genes order[g0 ..), boots of `pass` -- the
-// contraction kernel with one Q_BW-byte piece; S_twin: the twin joint's (a.W8_twin), or NULL.  prune_bound_ints(n_pos) ints.
+cudaError_t launch_z_bounds(const ContractI8Args &a, const double *Z, int n_sets, double *zb, cudaStream_t st);
+// each side's S[n_pos][104][Q_BW] = the sums of the drawn rows' bound rows (a.qbound) of genes order[g0 ..), boots of the
+// side -- the contraction kernel with one Q_BW-byte piece, over the sides s[0 .. n_sides).  prune_bound_ints(n_pos) ints.
 size_t prune_bound_ints(int n_pos);
-cudaError_t launch_bound_pass(const ContractI8Args &a, int g0, int n_pos, int pass, int n_sm, int32_t *S, int32_t *S_twin,
+cudaError_t launch_bound_pass(const ContractI8Args &a, int g0, int n_pos, const I8Side *s, int n_sides, int n_sm,
                               cudaStream_t st);
-// one joint's side of the decision: its sentinel ranges and bound sums of one launch, its Z extrema (first set, pass 0)
-struct PruneSide {
-    const uint32_t *sr;
-    const int32_t *S;
-    const double *zb;
-    int pass;
-};
-// live[pos] = the pieces not proven invisible for every boot of s0 (and of s1: a twin launch, where an item is contracted for
-// both joints); items / *n_live = the live items in launch order for launch_contract_i8_pass; stats (or NULL) [0] += items,
-// [1] += live items, [2] / [3] += the same weighted by the gene's list length.  live: n_pos bytes, items: n_pos *
-// q_pieces(K) ints.  lb_out [n_pos][104] / ub_out [n_pos][104][4] (tests, or NULL): s0's bounds (prune_decide_kernel).
-cudaError_t launch_prune_items(const ContractI8Args &a, int g0, int n_pos, const PruneSide &s0, const PruneSide *s1,
-                               uint8_t *live, int32_t *items, int32_t *n_live, unsigned long long *stats, cudaStream_t st,
+// live[pos] = the pieces not proven invisible for every boot of the sides s[0 .. n_sides) (from their sentinel ranges,
+// bound sums and Z extrema: an item of a two-sided launch is contracted for both); items / *n_live = the live items in
+// launch order for launch_contract_i8_pass; stats (or NULL) [0] += items, [1] += live items, [2] / [3] += the same
+// weighted by the gene's list length.  live: n_pos bytes, items: n_pos * q_pieces(K) ints.  lb_out [n_pos][104] / ub_out
+// [n_pos][104][4] (tests, or NULL): side 0's bounds (prune_decide_kernel).
+cudaError_t launch_prune_items(const ContractI8Args &a, int g0, int n_pos, const I8Side *s, int n_sides, uint8_t *live,
+                               int32_t *items, int32_t *n_live, unsigned long long *stats, cudaStream_t st,
                                double *lb_out = nullptr, double *ub_out = nullptr);
 // tests: out_host[0..3) = exp_nonpos(-745), (-746), (-747) on the device (synchronous on st's completion of the copy)
 cudaError_t launch_exp_probe(double *out_host, cudaStream_t st);
-// tests: turns the integer tiles in t_scratch into FP64 T (a.sentinel outside the ranges, no zero-count base), in place
-cudaError_t launch_finalize_t(const ContractI8Args &a, int n_pos, double *t_scratch, const uint32_t *sr, cudaStream_t st);
+// tests: turns the integer tiles in s.T into FP64 T (a.sentinel outside the ranges s.SR, no zero-count base), in place
+cudaError_t launch_finalize_t(const ContractI8Args &a, int n_pos, const I8Side &s, cudaStream_t st);
 
 // ---- ratio_summary.cu ----------------------------------------------------------------------------
 struct RatioContrast {  // one contrast of a batched launch: its joints and its outputs (layouts as in RatioArgs)

@@ -979,7 +979,13 @@ bool contract_i8_supported(int K, int ld_table, int ld_lst, int n_draws) {
 
 size_t contract_i8_range_words(int n_genes) { return (size_t)(n_genes > 0 ? n_genes : 1) * Q_WB; }
 
-static I8Params make_params(const ContractI8Args &a, int g0, int n_pos, int pass, double *t_scratch) {
+// boots of a side's pass
+static int side_boots(const ContractI8Args &a, const I8Side &s) {
+    return (a.n_boot - s.pass * WP_TILED) < WP_TILED ? (a.n_boot - s.pass * WP_TILED) : WP_TILED;
+}
+
+// the kernel's parameters of a launch over the sides s[0 .. n_sides): their W rows and T tiles, side 0's boots
+static I8Params make_params(const ContractI8Args &a, int g0, int n_pos, const I8Side *s, int n_sides) {
     I8Params p;
     p.qtable = a.qtable;
     p.ldq = a.ldq;
@@ -988,18 +994,18 @@ static I8Params make_params(const ContractI8Args &a, int g0, int n_pos, int pass
     p.lst_len = a.lists.len;
     p.order = a.lists.order ? a.lists.order + g0 : nullptr;
     p.ld_lst = a.lists.ld;
-    p.W8 = a.W8 + (size_t)pass * a.n_w_rows * Q_WB;
+    p.W8 = s[0].W8;
     p.gene_set = a.gene_set;
     p.set_w8 = a.set_w8;
-    p.T = reinterpret_cast<long long *>(t_scratch);
-    p.n_boot = (a.n_boot - pass * WP_TILED) < WP_TILED ? (a.n_boot - pass * WP_TILED) : WP_TILED;
+    p.T = reinterpret_cast<long long *>(s[0].T);
+    p.n_boot = side_boots(a, s[0]);
     p.n_pos = n_pos;
     p.n_pieces = q_pieces(a.K);
     p.err = a.err;
     p.dbg = a.dbg;
-    p.W8b = a.W8_twin ? a.W8_twin + (size_t)pass * a.n_w_rows * Q_WB : nullptr;
-    p.Tb = reinterpret_cast<long long *>(a.t_twin);
-    p.twin = (a.W8_twin && a.t_twin) ? 1 : 0;
+    p.W8b = n_sides > 1 ? s[1].W8 : nullptr;
+    p.Tb = n_sides > 1 ? reinterpret_cast<long long *>(s[1].T) : nullptr;
+    p.twin = n_sides > 1 ? 1 : 0;
     p.piece_major = a.item_order == 1;
     p.cold_evict_first = a.cold_evict_first;
     p.items = a.items;
@@ -1007,19 +1013,17 @@ static I8Params make_params(const ContractI8Args &a, int g0, int n_pos, int pass
     return p;
 }
 
-cudaError_t launch_sentinel_ranges(const ContractI8Args &a, int g0, int n_pos, int pass, uint32_t *sr_scratch,
-                                   cudaStream_t st) {
+cudaError_t launch_sentinel_ranges(const ContractI8Args &a, int g0, int n_pos, const I8Side &s, cudaStream_t st) {
     if (n_pos <= 0 || !a.row_range) return cudaSuccess;
-    if (!sr_scratch) return cudaErrorInvalidValue;
-    const I8Params p = make_params(a, g0, n_pos, pass, nullptr);
-    const int nb = (a.n_boot - pass * WP_TILED) < WP_TILED ? (a.n_boot - pass * WP_TILED) : WP_TILED;
+    if (!s.SR) return cudaErrorInvalidValue;
+    const I8Params p = make_params(a, g0, n_pos, &s, 1);
     sentinel_range_kernel<<<(unsigned)((n_pos + 7) / 8), 256, 0, st>>>(p.lst_row, p.lst_cell, p.lst_len, p.order, p.ld_lst,
                                                                        a.row_range, p.W8, a.gene_set, a.set_w8, n_pos, a.K,
-                                                                       nb, sr_scratch, a.err);
+                                                                       p.n_boot, s.SR, a.err);
     return cudaGetLastError();
 }
 
-cudaError_t launch_contract_i8_pass(const ContractI8Args &a, int g0, int n_pos, int pass, int n_sm, double *t_scratch,
+cudaError_t launch_contract_i8_pass(const ContractI8Args &a, int g0, int n_pos, const I8Side *s, int n_sides, int n_sm,
                                     cudaStream_t st) {
     if (n_pos <= 0) return cudaSuccess;
     // ONE producer group (four warps, one per k-group of a stage).  Round 1 used two groups that took alternate stages:
@@ -1030,7 +1034,7 @@ cudaError_t launch_contract_i8_pass(const ContractI8Args &a, int g0, int n_pos, 
     // next) that deadlocked scde.posteriors over 40 cells (tests: test_config2_..., test_short_and_long_lists_mixed...).
     // With one group every producer warp touches every stage, so the ring itself bounds its lead.
     constexpr int PG = 1;
-    const I8Params p = make_params(a, g0, n_pos, pass, t_scratch);
+    const I8Params p = make_params(a, g0, n_pos, s, n_sides);
     const int n_items = (n_pos * p.n_pieces) << p.twin;
     int grid = n_sm < n_items ? n_sm : n_items;
     if (p.twin) grid &= ~1;  // an even stride keeps every CTA on one joint and the pairs (2 i, 2 i + 1) together
@@ -1054,27 +1058,29 @@ size_t prune_zb_doubles(int n_sets, int n_boot) {
     return (size_t)(n_sets > 0 ? n_sets : 1) * (passes > 0 ? passes : 1) * WP_TILED * Q_BSLOTS;
 }
 
-cudaError_t launch_z_bounds(const ContractI8Args &a, int n_sets, double *zb, cudaStream_t st) {
+cudaError_t launch_z_bounds(const ContractI8Args &a, const double *Z, int n_sets, double *zb, cudaStream_t st) {
     const int64_t rows = (int64_t)prune_zb_doubles(n_sets, a.n_boot) / Q_BSLOTS;
-    z_bounds_kernel<<<(unsigned)((rows * Q_BSLOTS + 255) / 256), 256, 0, st>>>(a.Z, rows, a.K, zb);
+    z_bounds_kernel<<<(unsigned)((rows * Q_BSLOTS + 255) / 256), 256, 0, st>>>(Z, rows, a.K, zb);
     return cudaGetLastError();
 }
 
 size_t prune_bound_ints(int n_pos) { return (size_t)(n_pos > 0 ? n_pos : 1) * WP_TILED * Q_BW; }
 
-cudaError_t launch_bound_pass(const ContractI8Args &a, int g0, int n_pos, int pass, int n_sm, int32_t *S, int32_t *S_twin,
+cudaError_t launch_bound_pass(const ContractI8Args &a, int g0, int n_pos, const I8Side *s, int n_sides, int n_sm,
                               cudaStream_t st) {
     if (n_pos <= 0) return cudaSuccess;
     if (!a.qbound) return cudaErrorInvalidValue;
     constexpr int PG = 1;
-    ContractI8Args b = a;
-    b.items = nullptr;
-    b.t_twin = reinterpret_cast<double *>(S_twin);
-    I8Params p = make_params(b, g0, n_pos, pass, reinterpret_cast<double *>(S));
+    I8Params p = make_params(a, g0, n_pos, s, n_sides);
     p.qtable = a.qbound;
     p.ldq = Q_BW;
     p.n_pieces = 1;
     p.piece_major = 0;
+    p.items = nullptr;
+    p.n_live = nullptr;
+    // the BOUND kernel stores its int32 sums through T / Tb
+    p.T = reinterpret_cast<long long *>(s[0].S);
+    p.Tb = n_sides > 1 ? reinterpret_cast<long long *>(s[1].S) : nullptr;
     const int n_items = n_pos << p.twin;
     int grid = n_sm < n_items ? n_sm : n_items;
     if (p.twin) grid &= ~1;
@@ -1086,17 +1092,16 @@ cudaError_t launch_bound_pass(const ContractI8Args &a, int g0, int n_pos, int pa
     return cudaGetLastError();
 }
 
-cudaError_t launch_prune_items(const ContractI8Args &a, int g0, int n_pos, const PruneSide &s0, const PruneSide *s1,
-                               uint8_t *live, int32_t *items, int32_t *n_live, unsigned long long *stats, cudaStream_t st,
+cudaError_t launch_prune_items(const ContractI8Args &a, int g0, int n_pos, const I8Side *s, int n_sides, uint8_t *live,
+                               int32_t *items, int32_t *n_live, unsigned long long *stats, cudaStream_t st,
                                double *lb_out, double *ub_out) {
     if (n_pos <= 0) return cudaSuccess;
     const int32_t *order = a.lists.order ? a.lists.order + g0 : nullptr;
-    auto dev = [&](const PruneSide &s) {
-        return PruneSideDev{a.row_range ? s.sr : nullptr, s.S, s.zb + (size_t)s.pass * WP_TILED * Q_BSLOTS,
-                            (a.n_boot - s.pass * WP_TILED) < WP_TILED ? (a.n_boot - s.pass * WP_TILED) : WP_TILED};
+    auto dev = [&](const I8Side &x) {
+        return PruneSideDev{a.row_range ? x.SR : nullptr, x.S, x.zb + (size_t)x.pass * WP_TILED * Q_BSLOTS, side_boots(a, x)};
     };
     const int64_t set_zb = (int64_t)prune_zb_doubles(1, a.n_boot);
-    prune_decide_kernel<<<(unsigned)((n_pos + 7) / 8), 256, 0, st>>>(dev(s0), dev(s1 ? *s1 : s0), s1 ? 2 : 1, order,
+    prune_decide_kernel<<<(unsigned)((n_pos + 7) / 8), 256, 0, st>>>(dev(s[0]), dev(s[n_sides - 1]), n_sides, order,
                                                                      a.gene_set, set_zb, n_pos, a.K, q_pieces(a.K), live,
                                                                      lb_out, ub_out);
     cudaError_t e = cudaGetLastError();
@@ -1119,13 +1124,11 @@ cudaError_t launch_exp_probe(double *out_host, cudaStream_t st) {
 
 size_t softmax_i8_scratch_doubles(int n_pos) { return (size_t)SP_GROUPS * (n_pos > 0 ? n_pos : 1) * KP_TILED; }
 
-cudaError_t launch_softmax_i8(const ContractI8Args &a, int g0, int n_pos, int pass, const double *t_scratch, const uint32_t *sr,
-                              double *part_scratch, int n_sm, cudaStream_t st, const uint8_t *live) {
+cudaError_t launch_softmax_i8(const ContractI8Args &a, int g0, int n_pos, const I8Side &s, double *part_scratch, int n_sm,
+                              cudaStream_t st, const uint8_t *live) {
     if (n_pos <= 0) return cudaSuccess;
-    if (a.row_range && !sr) return cudaErrorInvalidValue;
-    const int nb = (a.n_boot - pass * WP_TILED) < WP_TILED ? (a.n_boot - pass * WP_TILED) : WP_TILED;
-    const double *Z = a.Z ? a.Z + (size_t)pass * WP_TILED * KP_TILED : nullptr;
-    const bool sets = a.gene_set && Z;
+    if (a.row_range && !s.SR) return cudaErrorInvalidValue;
+    const bool sets = a.gene_set && s.Z;
     const size_t smem = sets ? 0 : sizeof(double) * SP_ROWS * KP_TILED;
     auto kernel = sets ? (live ? softmax_i8_warp_kernel<true, true> : softmax_i8_warp_kernel<true, false>)
                        : (live ? softmax_i8_warp_kernel<false, true> : softmax_i8_warp_kernel<false, false>);
@@ -1134,23 +1137,23 @@ cudaError_t launch_softmax_i8(const ContractI8Args &a, int g0, int n_pos, int pa
     int wb = n_sm * 2 / SP_GROUPS;  // two CTAs of eight warps per SM
     if (wb * SW_WARPS > n_pos) wb = (n_pos + SW_WARPS - 1) / SW_WARPS;
     if (wb < 1) wb = 1;
-    kernel<<<wb * SP_GROUPS, SW_WARPS * 32, smem, st>>>(reinterpret_cast<const long long *>(t_scratch), Z,
-                                                        a.row_range ? sr : nullptr, a.K, nb, a.scale, part_scratch, n_pos,
-                                                        a.lists.order ? a.lists.order + g0 : nullptr, a.gene_set, a.set_z,
-                                                        live);
+    kernel<<<wb * SP_GROUPS, SW_WARPS * 32, smem, st>>>(reinterpret_cast<const long long *>(s.T), s.Z,
+                                                        a.row_range ? s.SR : nullptr, a.K, side_boots(a, s), a.scale,
+                                                        part_scratch, n_pos, a.lists.order ? a.lists.order + g0 : nullptr,
+                                                        a.gene_set, a.set_z, live);
     e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     const int64_t n = (int64_t)n_pos * KP_TILED;
     softmax_i8_reduce_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(part_scratch, a.lists.order ? a.lists.order + g0 : nullptr,
-                                                                          a.K, n_pos, a.jp, a.ld_jp, pass > 0);
+                                                                          a.K, n_pos, s.jp, a.ld_jp, s.pass > 0);
     return cudaGetLastError();
 }
 
-cudaError_t launch_finalize_t(const ContractI8Args &a, int n_pos, double *t_scratch, const uint32_t *sr, cudaStream_t st) {
+cudaError_t launch_finalize_t(const ContractI8Args &a, int n_pos, const I8Side &s, cudaStream_t st) {
     if (n_pos <= 0) return cudaSuccess;
     const int64_t n = (int64_t)n_pos * WP_TILED * KP_TILED;
-    finalize_t_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(reinterpret_cast<long long *>(t_scratch),
-                                                                   a.row_range ? sr : nullptr, a.sentinel, n);
+    finalize_t_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(reinterpret_cast<long long *>(s.T),
+                                                                   a.row_range ? s.SR : nullptr, a.sentinel, n);
     return cudaGetLastError();
 }
 
