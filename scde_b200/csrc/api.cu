@@ -398,7 +398,7 @@ int index_from_counts(scde_b200_ctx *ctx, LpTable &t, const int32_t *counts_dev,
 }
 
 // The device buffers of run_joint.  Joint j (W, Z, W8, zb): the j-th of the joints over the same cells that one run
-// computes together.  Side i (T, SR, S): the i-th side of a tcgen05 launch -- side 1 is the second joint, or the second
+// computes together.  Side i (T, SR): the i-th side of a tcgen05 launch -- side 1 is the second joint, or the second
 // pass of a paired-pass launch.
 struct JointScratch {
     DBuf<double> W[2], Z[2], T[2];
@@ -407,10 +407,9 @@ struct JointScratch {
     DBuf<uint32_t> SR[2];  // sentinel range of every (gene, boot) of one launch of the tcgen05 kernel
     DBuf<int32_t> lst_row, lst_cell, lst_len, order;
     DBuf<unsigned long long> total;  // running sums over the joints of one run: list lengths, then launch_prune_items' four
-    // pruning (launch_prune_items): Z extrema of each joint, bound sums of each side of one launch, live pieces and items
-    // of one launch, and the live count
+    // pruning (launch_prune_items): Z extrema of each joint, live pieces and items of one launch, and the live count
     DBuf<double> zb[2];
-    DBuf<int32_t> S[2], items, n_live;
+    DBuf<int32_t> items, n_live;
     DBuf<uint8_t> live;
 };
 
@@ -485,12 +484,11 @@ int contract_joint_i8(scde_b200_ctx *ctx, const LpTable &t, const GeneLists &lis
     for (int i = 0; i < n_sides; ++i) {
         SCDE_CUDA(scr.T[i].ensure(contract_tiled_scratch_doubles(t.n_genes)));
         SCDE_CUDA(scr.SR[i].ensure(contract_i8_range_words(mp)));
-        if (prune) SCDE_CUDA(scr.S[i].ensure(prune_bound_ints(mp)));
     }
     SCDE_CUDA(scr.spart.ensure(softmax_i8_scratch_doubles(mp)));
     if (prune) {
         for (int j = 0; j < n_joints; ++j) SCDE_CUDA(scr.zb[j].ensure(prune_zb_doubles(sets.n, n_boot)));
-        SCDE_CUDA(scr.live.ensure((size_t)mp));
+        SCDE_CUDA(scr.live.ensure(prune_live_bytes(mp)));
         SCDE_CUDA(scr.items.ensure((size_t)mp * q_pieces(t.K)));
         SCDE_CUDA(scr.n_live.ensure(1));
         q.qbound = t.qb.p;
@@ -499,7 +497,7 @@ int contract_joint_i8(scde_b200_ctx *ctx, const LpTable &t, const GeneLists &lis
     }
     auto side = [&](int j, int ps, int i) {  // joint j's pass ps as side i
         return I8Side{scr.W8[j].p + (size_t)ps * n_w_rows * Q_WB, scr.Z[j].p + (size_t)ps * WP_TILED * KP_TILED, scr.T[i].p,
-                      scr.SR[i].p, scr.S[i].p, scr.zb[j].p, joints[j].jp_dev, ps};
+                      scr.SR[i].p, scr.zb[j].p, joints[j].jp_dev, ps};
     };
     struct Launch {
         I8Side s[2];
@@ -529,9 +527,9 @@ int contract_joint_i8(scde_b200_ctx *ctx, const LpTable &t, const GeneLists &lis
             if (tm) tm->end(SCDE_B200_T_OTHER, e0, st, l.n);
             if (prune) {
                 e0 = tm ? tm->begin(st) : -1;
-                SCDE_CUDA(launch_bound_pass(q, g0, n_pos, l.s, l.n, ctx->n_sm, st));
-                SCDE_CUDA(launch_prune_items(q, g0, n_pos, l.s, l.n, scr.live.p, scr.items.p, scr.n_live.p, prune_stats, st));
-                if (tm) tm->end(SCDE_B200_T_BOUND, e0, st, 3);
+                SCDE_CUDA(launch_prune_items(q, g0, n_pos, l.s, l.n, ctx->n_sm, scr.live.p, scr.items.p, scr.n_live.p,
+                                             prune_stats, st));
+                if (tm) tm->end(SCDE_B200_T_BOUND, e0, st, 2);
             }
             e0 = tm ? tm->begin(st) : -1;
             SCDE_CUDA(launch_contract_i8_pass(q, g0, n_pos, l.s, l.n, ctx->n_sm, st));
@@ -1942,28 +1940,26 @@ int scde_b200_probe_prune_i8(scde_b200_ctx *ctx, const int8_t *qtable, int32_t n
     q.hot_rank = -1;
     q.cold_evict_first = 0;
     q.ring_stages = ctx->opt.ring_stages;
-    I8Side side{d_w.p, nullptr, d_t.p, d_sr.p, nullptr, nullptr, nullptr, 0};
+    I8Side side{d_w.p, nullptr, d_t.p, d_sr.p, nullptr, nullptr, 0};
     SCDE_CUDA(launch_sentinel_ranges(q, 0, n_genes, side, st));
     DBuf<int8_t> d_qb;
     DBuf<double> d_z, d_zb, d_lb, d_ub;
-    DBuf<int32_t> d_s, d_items, d_nlive;
+    DBuf<int32_t> d_items, d_nlive;
     DBuf<uint8_t> d_live;
     if (qbound) {  // the decision of the pruned contraction, with its bounds; T itself is contracted unpruned
         TRY(upload(d_qb, qbound, (size_t)n_rows * Q_BW, st));
         if (z) TRY(upload(d_z, z, (size_t)WP_TILED * KP_TILED, st));
         q.qbound = d_qb.p;
         SCDE_CUDA(d_zb.ensure(prune_zb_doubles(1, WP_TILED)));
-        SCDE_CUDA(d_s.ensure(prune_bound_ints(n_genes)));
         SCDE_CUDA(d_lb.ensure((size_t)n_genes * WP_TILED));
         SCDE_CUDA(d_ub.ensure((size_t)n_genes * WP_TILED * 4));
-        SCDE_CUDA(d_live.ensure((size_t)n_genes));
+        SCDE_CUDA(d_live.ensure(prune_live_bytes(n_genes)));
         SCDE_CUDA(d_items.ensure((size_t)n_genes * q_pieces(n_grid)));
         SCDE_CUDA(d_nlive.ensure(1));
-        side.S = d_s.p;
         side.zb = d_zb.p;
         SCDE_CUDA(launch_z_bounds(q, z ? d_z.p : nullptr, 1, d_zb.p, st));
-        SCDE_CUDA(launch_bound_pass(q, 0, n_genes, &side, 1, ctx->n_sm, st));
-        SCDE_CUDA(launch_prune_items(q, 0, n_genes, &side, 1, d_live.p, d_items.p, d_nlive.p, nullptr, st, d_lb.p, d_ub.p));
+        SCDE_CUDA(launch_prune_items(q, 0, n_genes, &side, 1, ctx->n_sm, d_live.p, d_items.p, d_nlive.p, nullptr, st, d_lb.p,
+                                     d_ub.p));
     }
     SCDE_CUDA(launch_contract_i8_pass(q, 0, n_genes, &side, 1, ctx->n_sm, st));
     SCDE_CUDA(launch_finalize_t(q, n_genes, side, st));

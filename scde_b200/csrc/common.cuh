@@ -257,7 +257,7 @@ struct ContractI8Args {
                        // rows are loaded with the L2 evict_last policy, the others evict_first.  < 0: no hints
     int cold_evict_first;  // with hot_rank >= 0: 1 = the other rows are loaded evict_first, 0 = without a priority
     int ring_stages;       // 0 / 10: the full 10-stage ring (200 KB in flight per SM); 7 or 8: a shallower one
-    const int8_t *qbound;  // the table's bound rows [rows][Q_BW] (launch_bound_pass)
+    const int8_t *qbound;  // the table's bound rows [rows][Q_BW] (launch_prune_items)
     const int32_t *items;  // launch_contract_i8_pass: contract only the live items, items[0 .. *n_live) (launch_prune_items);
     const int32_t *n_live; // NULL = every item
 };
@@ -270,7 +270,6 @@ struct I8Side {
     const double *Z;    // the pass's base sums [104][416] of the first draw set, or NULL
     double *T;          // T tiles [n_pos][104][416] of one launch
     uint32_t *SR;       // sentinel ranges [n_pos][128] of one launch
-    int32_t *S;         // bound sums [n_pos][104][Q_BW] of one launch (pruning)
     const double *zb;   // the joint's Z extrema (launch_z_bounds; pruning)
     double *jp;         // the joint's output [n_genes][ld_jp]
     int pass;
@@ -299,17 +298,13 @@ cudaError_t launch_softmax_i8(const ContractI8Args &a, int g0, int n_pos, const 
 // zb: prune_zb_doubles() doubles, the Z extrema of every (set, pass, boot) of a joint (its Z, a.n_boot, a.K), once per joint
 size_t prune_zb_doubles(int n_sets, int n_boot);
 cudaError_t launch_z_bounds(const ContractI8Args &a, const double *Z, int n_sets, double *zb, cudaStream_t st);
-// each side's S[n_pos][104][Q_BW] = the sums of the drawn rows' bound rows (a.qbound) of genes order[g0 ..), boots of the
-// side -- the contraction kernel with one Q_BW-byte piece, over the sides s[0 .. n_sides).  prune_bound_ints(n_pos) ints.
-size_t prune_bound_ints(int n_pos);
-cudaError_t launch_bound_pass(const ContractI8Args &a, int g0, int n_pos, const I8Side *s, int n_sides, int n_sm,
-                              cudaStream_t st);
-// live[pos] = the pieces not proven invisible for every boot of the sides s[0 .. n_sides) (from their sentinel ranges,
-// bound sums and Z extrema: an item of a two-sided launch is contracted for both); items / *n_live = the live items in
-// launch order for launch_contract_i8_pass; stats (or NULL) [0] += items, [1] += live items, [2] / [3] += the same
-// weighted by the gene's list length.  live: n_pos bytes, items: n_pos * q_pieces(K) ints.  lb_out [n_pos][104] / ub_out
-// [n_pos][104][4] (tests, or NULL): side 0's bounds (prune_decide_kernel).
-cudaError_t launch_prune_items(const ContractI8Args &a, int g0, int n_pos, const I8Side *s, int n_sides, uint8_t *live,
+// live[pos] = the pieces not proven invisible for every boot of the sides s[0 .. n_sides) (bound_i8_kernel: the sums of
+// the drawn rows' bound rows a.qbound, with the sentinel ranges and Z extrema of each side; an item of a two-sided launch
+// is contracted for both); items / *n_live = the live items in launch order for launch_contract_i8_pass; stats (or NULL)
+// [0] += items, [1] += live items, [2] / [3] += the same weighted by the gene's list length.  live: prune_live_bytes(n_pos)
+// bytes, items: n_pos * q_pieces(K) ints.  lb_out [n_pos][104] / ub_out [n_pos][104][4] (tests, or NULL): side 0's bounds.
+size_t prune_live_bytes(int n_pos);
+cudaError_t launch_prune_items(const ContractI8Args &a, int g0, int n_pos, const I8Side *s, int n_sides, int n_sm, uint8_t *live,
                                int32_t *items, int32_t *n_live, unsigned long long *stats, cudaStream_t st,
                                double *lb_out = nullptr, double *ub_out = nullptr);
 // tests: out_host[0..3) = exp_nonpos(-745), (-746), (-747) on the device (synchronous on st's completion of the copy)

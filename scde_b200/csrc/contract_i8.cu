@@ -100,7 +100,8 @@ struct I8Params {
     const int32_t *n_live; // them, written on the device by prune_compact_kernel; NULL = every item
 };
 
-__device__ __forceinline__ bool wait_or_abort(I8Smem &sm, uint64_t *bar, uint32_t parity) {
+template <class Smem>
+__device__ __forceinline__ bool wait_or_abort(Smem &sm, uint64_t *bar, uint32_t parity) {
     if (mbar_try_wait(bar, parity)) return true;
     const long long t0 = clock64();
     while (!mbar_try_wait(bar, parity)) {
@@ -169,8 +170,7 @@ __device__ __forceinline__ void cp_async16_hint_at(uint32_t dst_smem, const void
 // HINT: list entries carry LIST_HOT_BIT in `cell` when the row is one of the first few of its cell (a small count: such a
 // row is shared by thousands of genes); its pieces are loaded with the L2 evict_last policy, the others evict_first (or
 // unhinted), so that the stream of rows that are used once does not push the shared ones out of the L2.
-// BOUND: the bound pass -- one Q_BW-byte piece per row (p.qtable = the bound rows), one 128-byte run per entry.
-template <int Q_PGROUPS, bool HINT, int NS, bool BOUND>
+template <int Q_PGROUPS, bool HINT, int NS>
 __device__ __forceinline__ void run_producer(const I8Params &p, I8Smem &sm, uint32_t stage0, int n_items, int warp, int lane) {
     uint64_t pol_hot = 0, pol_cold = 0;
     if (HINT) {
@@ -204,7 +204,7 @@ __device__ __forceinline__ void run_producer(const I8Params &p, I8Smem &sm, uint
             len_n = p.lst_len[gene_n];
             if (p.gene_set) wset_n = p.gene_set[gene_n] * p.set_w8;
         }
-        const int8_t *qbase = p.qtable + (BOUND ? 0 : (int64_t)it.piece * Q_PIECE) + l7 * 16;
+        const int8_t *qbase = p.qtable + (int64_t)it.piece * Q_PIECE + l7 * 16;
         const int8_t *wbase = ((p.twin && (item & 1)) ? p.W8b : p.W8) + l7 * 16 + wset;
         const int32_t *lrow = p.lst_row + gene * p.ld_lst + kg * 8 + l3;
         const int32_t *lcell = p.lst_cell + gene * p.ld_lst + kg * 8 + l3;
@@ -242,12 +242,7 @@ __device__ __forceinline__ void run_producer(const I8Params &p, I8Smem &sm, uint
                     const int8_t *w0 = wbase + (int64_t)(cel0 & ~LIST_HOT_BIT) * Q_WB;
                     const int8_t *w1 = wbase + (int64_t)(cel1 & ~LIST_HOT_BIT) * Q_WB;
                     if (fill > 0 && !wait_or_abort(sm, &sm.empty[slot], (fill - 1) & 1u)) return;
-                    if (BOUND) {
-                        cp_async16_at<0, 0>(sB0, src0);
-                        cp_async16_at<0, 0>(sB1, src1);
-                        cp_async16_at<0, 0>(sA + d0, w0);
-                        cp_async16_at<0, 0>(sA + d1, w1);
-                    } else if (HINT) {
+                    if (HINT) {
                         const uint64_t pol0 = (cel0 & LIST_HOT_BIT) ? pol_hot : pol_cold;
                         const uint64_t pol1 = (cel1 & LIST_HOT_BIT) ? pol_hot : pol_cold;
                         cp_async16_hint_at<0, 0>(sB0, src0, pol0);
@@ -296,9 +291,9 @@ __device__ __forceinline__ void run_producer(const I8Params &p, I8Smem &sm, uint
 }
 
 // ---- MMA issuer (one thread) ------------------------------------------------------------------------------------------
-template <int NS, bool BOUND>
+template <int NS>
 __device__ __forceinline__ void run_mma(const I8Params &p, I8Smem &sm, uint32_t stage0, uint32_t tmem, int n_items) {
-    const uint32_t idesc = umma_idesc_s8_mn(128, BOUND ? Q_BW : 256);
+    const uint32_t idesc = umma_idesc_s8_mn(128, 256);
     int slot = 0;
     uint32_t fill = 0, n_done = 0;
     int item = blockIdx.x;
@@ -320,7 +315,7 @@ __device__ __forceinline__ void run_mma(const I8Params &p, I8Smem &sm, uint32_t 
             const uint32_t sB = sA + Q_A_BYTES;
             const uint64_t da = umma_desc_sw128(sA, 4096u, 1024u);
             umma_s8(tmem, da, umma_desc_sw128(sB, 4096u, 1024u), idesc, s > 0);                      // runs 0, 1
-            if (!BOUND) umma_s8(tmem + 256u, da, umma_desc_sw128(sB + 2u * 4096u, 4096u, 1024u), idesc, s > 0);  // runs 2, 3
+            umma_s8(tmem + 256u, da, umma_desc_sw128(sB + 2u * 4096u, 4096u, 1024u), idesc, s > 0);  // runs 2, 3
             umma_commit(&sm.empty[slot]);  // frees the slot once these MMAs have read it
             if (++slot == NS) {
                 slot = 0;
@@ -416,40 +411,7 @@ __device__ __forceinline__ void run_epilogue(const I8Params &p, I8Smem &sm, uint
     }
 }
 
-// bound pass: the 128 int32 sums of a (gene, boot), stored as they are (p.T / p.Tb: [n_pos][104][Q_BW]); warp e reads the
-// lanes of quarter e & 3 and the columns 64 (e >> 2) .. + 63
-__device__ __forceinline__ void run_bound_epilogue(const I8Params &p, I8Smem &sm, uint32_t tmem, int n_items, int ewarp, int lane) {
-    const int qd = ewarp & 3, half = ewarp >> 2;
-    const uint32_t tcol = tmem + ((uint32_t)(qd * 32) << 16) + (uint32_t)(half * 64);
-    const int boot = qd * 32 + lane;
-    uint32_t n_done = 0;
-    for (int item = blockIdx.x; item < n_items; item += gridDim.x, ++n_done) {
-        const int pos = item >> p.twin;
-        const bool empty_list = p.lst_len[p.order ? p.order[pos] : pos] <= 0;
-        while (!mbar_try_wait(&sm.acc_full, n_done & 1u)) {
-            __nanosleep(200);
-            if (sm.abort) return;
-        }
-        tc_fence_after_sync();
-        int4 *dst = reinterpret_cast<int4 *>(reinterpret_cast<int32_t *>((p.twin && (item & 1)) ? p.Tb : p.T) +
-                                             ((int64_t)pos * WP_TILED + boot) * Q_BW + half * 64);
-        for (int c = 0; c < 64; c += 8) {
-            uint32_t r[8] = {0u, 0u, 0u, 0u, 0u, 0u, 0u, 0u};
-            if (!empty_list) {
-                tmem_ld_32x32b_x8(tcol + (uint32_t)c, r);
-                tmem_wait_ld();
-            }
-            if (boot < p.n_boot) {
-                dst[c / 4] = make_int4((int)r[0], (int)r[1], (int)r[2], (int)r[3]);
-                dst[c / 4 + 1] = make_int4((int)r[4], (int)r[5], (int)r[6], (int)r[7]);
-            }
-        }
-        tc_fence_before_sync();
-        mbar_arrive(&sm.acc_empty);
-    }
-}
-
-template <int Q_PGROUPS, bool HINT, int NS, bool BOUND>
+template <int Q_PGROUPS, bool HINT, int NS>
 __global__ void __launch_bounds__(q_threads(Q_PGROUPS), 1) contract_i8_kernel(const I8Params p) {
     static_assert(NS >= 2 && NS <= Q_NS, "ring depth");
     constexpr int Q_PRODUCER_WARPS = 4 * Q_PGROUPS;
@@ -478,14 +440,11 @@ __global__ void __launch_bounds__(q_threads(Q_PGROUPS), 1) contract_i8_kernel(co
     const int n_items = (p.items ? *p.n_live : p.n_pos * p.n_pieces) << p.twin;
 
     if (warp < Q_PRODUCER_WARPS)
-        run_producer<Q_PGROUPS, HINT, NS, BOUND>(p, sm, stage0, n_items, warp, lane);
-    else if (warp < Q_PRODUCER_WARPS + Q_EPILOGUE_WARPS) {
-        if (BOUND)
-            run_bound_epilogue(p, sm, tmem, n_items, warp - Q_PRODUCER_WARPS, lane);
-        else
-            run_epilogue(p, sm, xbuf, tmem, n_items, warp - Q_PRODUCER_WARPS, lane);
-    } else if (lane == 0)
-        run_mma<NS, BOUND>(p, sm, stage0, tmem, n_items);
+        run_producer<Q_PGROUPS, HINT, NS>(p, sm, stage0, n_items, warp, lane);
+    else if (warp < Q_PRODUCER_WARPS + Q_EPILOGUE_WARPS)
+        run_epilogue(p, sm, xbuf, tmem, n_items, warp - Q_PRODUCER_WARPS, lane);
+    else if (lane == 0)
+        run_mma<NS>(p, sm, stage0, tmem, n_items);
 
     tc_fence_before_sync();
     __syncthreads();
@@ -604,7 +563,7 @@ static_assert(SP_GROUPS * SP_ROWS == WP_TILED && SP_ROWS * 32 == KP_TILED, "13 w
 // SETS (several draw sets, DESIGN.md "Draw sets"): each gene reads the Z rows of its own set, gene_set[gene] * set_z doubles
 // after Z, from global memory (L2) instead of shared memory -- the same values in the same order, so the same result.
 // live (pruned launches, else NULL): bit p of live[pos] = piece p of the gene was contracted.  The points of the other
-// pieces are neither loaded (their T tiles were not written) nor candidates: prune_decide_kernel proved them more than
+// pieces are neither loaded (their T tiles were not written) nor candidates: bound_i8_kernel proved them more than
 // 746 nats below the row maximum for every boot, where exp_nonpos is exactly 0 -- m, sum, amask and acc are unchanged.
 constexpr int SW_WARPS = 8;
 // LIVE: the instance of pruned launches (live != NULL); the other one is the kernel as it was before pruning.
@@ -751,58 +710,333 @@ __global__ void z_bounds_kernel(const double *__restrict__ Z, int64_t n_rows, in
     zb[idx] = v;
 }
 
-// one warp per gene: live[pos] = the pieces that are not dead for the boots of side 0 (and of side 1: twin launches)
-struct PruneSideDev {
-    const uint32_t *sr;
-    const int32_t *S;
-    const double *zb;
-    int n_boot;
+// ---- bound_i8_kernel: the bound sums and the decision in one pass -------------------------------------------------------
+// live[pos] = the pieces of gene order[pos] that are not dead for every real boot of the launch's sides.  Persistent, one
+// CTA per SM, item = one gene with both sides of a two-sided launch, the contraction kernel's three warp roles in a
+// geometry of its own:
+//   * producers (4 warps, one group: the ring bounds their lead, see launch_contract_i8_pass): a stage is 32 list
+//     entries -- each side's 128-byte W rows and, gathered ONCE for both sides, the 128-byte bound rows -- copied with
+//     16-byte cp.async into the 128-byte-swizzle layout (the contraction's producer loop).  B_RING = 192 KB of 8 or 12 KB
+//     stages are in flight per SM; the contraction's ring, whose 20 KB stages a bound stage filled only 8 KB of, held 80.
+//   * MMA (1 thread): per stage and side one tcgen05.mma (M = 128 boots, N = 128 bound columns, K = 32 entries) into the
+//     side's accumulator of the gene's buffer.  The 512 tensor-memory columns hold 4 buffers (one side) or 2 (two), each
+//     with its own full / empty barrier, so the MMAs of the next genes run while the epilogue reads this one.
+//   * epilogue (8 warps): a thread owns one boot (tensor-memory lane) of its warp's quarter.  The warps of half 1 form LB
+//     from the sample slots, those of half 0 UB_p from the block slots -- both digits of a slot in one thread -- with the
+//     arithmetic of the formulas above; LB reaches the UB thread of its boot through shared memory.  The dead pieces are
+//     ANDed over the sides and the warp's boots, and each warp ORs its live pieces into live[pos] (zeroed before the
+//     launch).  The sums never leave the SM.
+constexpr int B_TILE = Q_ES * Q_WB;  // one operand tile of a stage: 32 entries x 128 bytes = 4096
+constexpr int B_RING = 192 * 1024;
+template <int SIDES>
+struct BoundGeom {
+    static constexpr int STAGE = (SIDES + 1) * B_TILE;            // the sides' W tiles, then the bound-row tile
+    static constexpr int NS = B_RING / STAGE;                     // 24 or 16 stages
+    static constexpr int NACC = Q_TMEM_COLS / (SIDES * Q_BW);     // accumulator buffers: 4 or 2
 };
-__global__ void __launch_bounds__(256) prune_decide_kernel(PruneSideDev s0, PruneSideDev s1, int sides, const int32_t *__restrict__ order,
-                                                           const int32_t *__restrict__ gene_set, int64_t set_zb, int n_pos, int K,
-                                                           int n_pieces, uint8_t *__restrict__ live, double *__restrict__ lb_out,
-                                                           double *__restrict__ ub_out) {
-    const int pos = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    if (pos >= n_pos) return;
-    const int lane = threadIdx.x & 31;
-    const int64_t zoff = gene_set ? gene_set[order ? order[pos] : pos] * set_zb : 0;
-    const uint32_t all = (1u << n_pieces) - 1u;
-    uint32_t dead = all;
-    for (int side = 0; side < sides; ++side) {
-        const PruneSideDev s = side ? s1 : s0;
-        for (int b = lane; b < s.n_boot; b += 32) {
-            const uint32_t sr = s.sr ? s.sr[(int64_t)pos * Q_WB + b] : 0xFFFF0000u;
-            const int klo = (int)(sr & 0xFFFFu), khi = min((int)(sr >> 16), K - 1);
-            const int32_t *S = s.S + ((int64_t)pos * WP_TILED + b) * Q_BW;
-            const double *z = s.zb + zoff + (int64_t)b * Q_BSLOTS;
-            double lb = -INFINITY;
-            for (int c = 0; c < Q_LB_N; ++c) {
-                const int k = Q_LB_STEP * c + Q_LB_OFF;
-                if (k >= klo && k <= khi)
-                    lb = fmax(lb, z[Q_UB_N + c] + ((double)S[Q_UB_N + c] + 256.0 * S[Q_BSLOTS + Q_UB_N + c]) * (1.0 / 32.0));
+template <int SIDES>
+struct BoundSmem {
+    uint64_t full[BoundGeom<SIDES>::NS], empty[BoundGeom<SIDES>::NS];
+    uint64_t acc_full[BoundGeom<SIDES>::NACC], acc_empty[BoundGeom<SIDES>::NACC];
+    uint64_t lb_full, lb_empty;  // the LB exchange: written by half 1, read by half 0
+    double lb[SIDES][Q_WB];
+    uint32_t tmem_base;
+    volatile int abort;
+};
+template <int SIDES>
+constexpr size_t bound_smem_bytes() { return 1024 /* alignment slack */ + (size_t)B_RING + sizeof(BoundSmem<SIDES>); }
+
+struct BoundParams {
+    const int8_t *qbound;  // the table's bound rows [rows][Q_BW]
+    const int32_t *lst_row, *lst_cell, *lst_len, *order;
+    int64_t ld_lst;
+    const int32_t *gene_set;  // draw set of every gene (NULL: one set)
+    int64_t set_w8, set_zb;   // bytes of W8 / doubles of zb per draw set
+    const int8_t *W8[2];      // side s: its pass's W rows [n_w_rows][128] (of the first draw set)
+    const uint32_t *SR[2];    // side s: sentinel ranges [n_pos][128], or NULL (no row holds a sentinel)
+    const double *zb[2];      // side s: its pass's Z extrema [104][Q_BSLOTS] (of the first draw set)
+    int n_boot[2];            // side s: real boots
+    int n_pos, K, n_pieces;
+    uint32_t *live;           // live[pos] (bytes), written as words by atomicOr
+    double *lb_out, *ub_out;  // side 0's LB [n_pos][104] and UB [n_pos][104][4] (scde_b200_probe_prune_i8), or NULL
+};
+
+template <int SIDES>
+__device__ __forceinline__ void bound_producer(const BoundParams &p, BoundSmem<SIDES> &sm, uint32_t stage0, int warp, int lane) {
+    using G = BoundGeom<SIDES>;
+    const int kg = warp, l7 = lane & 7, l3 = lane >> 3;
+    const uint32_t d0 = (uint32_t)kg * 1024u + (uint32_t)l3 * 128u + (uint32_t)((l7 ^ l3) << 4);
+    const uint32_t d1 = (uint32_t)kg * 1024u + (uint32_t)(l3 + 4) * 128u + (uint32_t)((l7 ^ (l3 + 4)) << 4);
+    int slot = 0;
+    uint32_t fill = 0;
+    int pos = blockIdx.x;
+    int64_t gene_n = 0, wset_n = 0;
+    int len_n = 0;
+    if (pos < p.n_pos) {
+        gene_n = p.order ? p.order[pos] : pos;
+        len_n = p.lst_len[gene_n];
+        if (p.gene_set) wset_n = p.gene_set[gene_n] * p.set_w8;
+    }
+    for (; pos < p.n_pos; pos += gridDim.x) {
+        const int64_t gene = gene_n, wset = wset_n;
+        const int nst = (len_n + Q_ES - 1) / Q_ES;
+        if (pos + (int)gridDim.x < p.n_pos) {
+            gene_n = p.order ? p.order[pos + gridDim.x] : pos + gridDim.x;
+            len_n = p.lst_len[gene_n];
+            if (p.gene_set) wset_n = p.gene_set[gene_n] * p.set_w8;
+        }
+        const int8_t *qbase = p.qbound + l7 * 16;
+        const int8_t *wb0 = p.W8[0] + wset + l7 * 16;
+        const int8_t *wb1 = p.W8[SIDES - 1] + wset + l7 * 16;
+        const int32_t *lrow = p.lst_row + gene * p.ld_lst + kg * 8 + l3;
+        const int32_t *lcell = p.lst_cell + gene * p.ld_lst + kg * 8 + l3;
+        int32_t r0a = 0, r1a = 0, c0a = 0, c1a = 0, r0b = 0, r1b = 0, c0b = 0, c1b = 0;
+        auto load_block = [&](int t, int32_t &r0, int32_t &r1, int32_t &c0, int32_t &c1) {
+            const int s = 8 * t + l7;
+            r0 = r1 = c0 = c1 = 0;
+            if (s < nst) {
+                r0 = __ldg(lrow + s * Q_ES);
+                r1 = __ldg(lrow + s * Q_ES + 4);
+                c0 = __ldg(lcell + s * Q_ES);
+                c1 = __ldg(lcell + s * Q_ES + 4);
             }
-            double ub[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
-            for (int u = 0; u < Q_UB_N; ++u) {
-                const int lo = max(u * Q_UB_PTS, klo), hi = min(u * Q_UB_PTS + Q_UB_PTS - 1, khi);
-                if (lo > hi) continue;
-                const double v = z[u] + ((double)S[u] + 256.0 * S[Q_BSLOTS + u]) * (1.0 / 32.0);
+        };
+        load_block(0, r0a, r1a, c0a, c1a);
+        load_block(1, r0b, r1b, c0b, c1b);
+        for (int t = 0; 8 * t < nst; ++t) {
 #pragma unroll
-                for (int pc = 0; pc < 4; ++pc)
-                    if (max(lo, pc * Q_PW) <= min(hi, pc * Q_PW + Q_PW - 1)) ub[pc] = fmax(ub[pc], v);
+            for (int u = 0; u < 8; ++u) {
+                if (8 * t + u < nst) {  // warp-uniform
+                    const int from = (lane & 24) | u;
+                    const int32_t row0 = __shfl_sync(0xffffffffu, r0a, from), row1 = __shfl_sync(0xffffffffu, r1a, from);
+                    const int64_t cel0 = __shfl_sync(0xffffffffu, c0a, from) & ~LIST_HOT_BIT;
+                    const int64_t cel1 = __shfl_sync(0xffffffffu, c1a, from) & ~LIST_HOT_BIT;
+                    const uint32_t sA = stage0 + (uint32_t)slot * G::STAGE, sB = sA + SIDES * B_TILE;
+                    if (fill > 0 && !wait_or_abort(sm, &sm.empty[slot], (fill - 1) & 1u)) return;
+                    cp_async16_at<0, 0>(sB + d0, qbase + (int64_t)row0 * Q_BW);
+                    cp_async16_at<0, 0>(sB + d1, qbase + (int64_t)row1 * Q_BW);
+                    cp_async16_at<0, 0>(sA + d0, wb0 + cel0 * Q_WB);
+                    cp_async16_at<0, 0>(sA + d1, wb0 + cel1 * Q_WB);
+                    if (SIDES > 1) {
+                        cp_async16_at<B_TILE, 0>(sA + d0, wb1 + cel0 * Q_WB);
+                        cp_async16_at<B_TILE, 0>(sA + d1, wb1 + cel1 * Q_WB);
+                    }
+                    cp_async_mbar_arrive_noinc(&sm.full[slot]);
+                    if (++slot == G::NS) {
+                        slot = 0;
+                        ++fill;
+                    }
+                }
             }
-            if (lb_out && side == 0) {  // scde_b200_probe_prune_i8
-                lb_out[(int64_t)pos * WP_TILED + b] = lb;
-                for (int pc = 0; pc < 4; ++pc) ub_out[((int64_t)pos * WP_TILED + b) * 4 + pc] = ub[pc];
-            }
-            const double thr = lb - 747.0;  // lb = -inf (no sample inside the range): nothing is dead
-            uint32_t d = 0u;
-#pragma unroll
-            for (int pc = 0; pc < 4; ++pc) d |= ub[pc] < thr ? 1u << pc : 0u;
-            dead &= d;
+            r0a = r0b;
+            r1a = r1b;
+            c0a = c0b;
+            c1a = c1b;
+            load_block(t + 2, r0b, r1b, c0b, c1b);
         }
     }
-    dead = __reduce_and_sync(0xffffffffu, dead);
-    if (lane == 0) live[pos] = (uint8_t)(~dead & all);
+}
+
+template <int SIDES>
+__device__ __forceinline__ void bound_mma(const BoundParams &p, BoundSmem<SIDES> &sm, uint32_t stage0, uint32_t tmem) {
+    using G = BoundGeom<SIDES>;
+    const uint32_t idesc = umma_idesc_s8_mn(128, Q_BW);
+    int slot = 0;
+    uint32_t fill = 0, n_done = 0;
+    int pos = blockIdx.x;
+    int len_n = pos < p.n_pos ? p.lst_len[p.order ? p.order[pos] : pos] : 0;
+    for (; pos < p.n_pos; pos += gridDim.x, ++n_done) {
+        const int nst = (len_n + Q_ES - 1) / Q_ES;
+        if (pos + (int)gridDim.x < p.n_pos) len_n = p.lst_len[p.order ? p.order[pos + gridDim.x] : pos + gridDim.x];
+        const int buf = (int)(n_done % G::NACC);
+        const uint32_t use = n_done / G::NACC;
+        if (use > 0) {  // the epilogue has read this buffer's previous gene
+            if (!wait_or_abort(sm, &sm.acc_empty[buf], (use - 1) & 1u)) return;
+            tc_fence_after_sync();
+        }
+        const uint32_t acc = tmem + (uint32_t)(buf * SIDES * Q_BW);
+        for (int s = 0; s < nst; ++s) {
+            if (!wait_or_abort(sm, &sm.full[slot], fill & 1u)) return;
+            fence_proxy_async_smem();
+            tc_fence_after_sync();
+            const uint32_t sA = stage0 + (uint32_t)slot * G::STAGE;
+            const uint64_t db = umma_desc_sw128(sA + SIDES * B_TILE, 4096u, 1024u);
+#pragma unroll
+            for (int side = 0; side < SIDES; ++side)
+                umma_s8(acc + (uint32_t)(side * Q_BW), umma_desc_sw128(sA + side * B_TILE, 4096u, 1024u), db, idesc, s > 0);
+            umma_commit(&sm.empty[slot]);
+            if (++slot == G::NS) {
+                slot = 0;
+                ++fill;
+            }
+        }
+        if (nst > 0)
+            umma_commit(&sm.acc_full[buf]);
+        else
+            mbar_arrive(&sm.acc_full[buf]);  // an empty list: the sums are 0, nothing to wait for
+    }
+}
+
+// the epilogue's waits: a gene takes microseconds, so sleep between polls; false when the kernel aborts
+template <int SIDES>
+__device__ __forceinline__ bool bound_wait(BoundSmem<SIDES> &sm, uint64_t *bar, uint32_t parity) {
+    while (!mbar_try_wait(bar, parity)) {
+        __nanosleep(100);
+        if (sm.abort) return false;
+    }
+    return true;
+}
+
+template <int SIDES>
+__device__ __forceinline__ void bound_epilogue(const BoundParams &p, BoundSmem<SIDES> &sm, uint32_t tmem, int ewarp, int lane) {
+    using G = BoundGeom<SIDES>;
+    const int qd = ewarp & 3, half = ewarp >> 2;
+    const int boot = qd * 32 + lane;
+    const uint32_t tq = tmem + ((uint32_t)(qd * 32) << 16);
+    const uint32_t all = (1u << p.n_pieces) - 1u;
+    uint32_t n_done = 0;
+    for (int pos = blockIdx.x; pos < p.n_pos; pos += gridDim.x, ++n_done) {
+        const int64_t gene = p.order ? p.order[pos] : pos;
+        const bool empty_list = p.lst_len[gene] <= 0;
+        const int64_t zoff = p.gene_set ? p.gene_set[gene] * p.set_zb : 0;
+        int klo[SIDES], khi[SIDES];
+        const double *zr[SIDES];
+#pragma unroll
+        for (int side = 0; side < SIDES; ++side) {
+            const uint32_t sr = p.SR[side] ? p.SR[side][(int64_t)pos * Q_WB + boot] : 0xFFFF0000u;
+            klo[side] = (int)(sr & 0xFFFFu);
+            khi[side] = min((int)(sr >> 16), p.K - 1);
+            zr[side] = p.zb[side] + zoff + (int64_t)(boot < p.n_boot[side] ? boot : 0) * Q_BSLOTS;  // past the boots: not used
+        }
+        const int buf = (int)(n_done % G::NACC);
+        if (!bound_wait(sm, &sm.acc_full[buf], (n_done / G::NACC) & 1u)) return;
+        tc_fence_after_sync();
+        // slot i of the bound row: digits in columns i and Q_BSLOTS + i, read 8 slots at a time
+        auto load8 = [&](int side, int j, uint32_t (&lo)[8], uint32_t (&hi)[8]) {
+#pragma unroll
+            for (int i = 0; i < 8; ++i) lo[i] = hi[i] = 0u;
+            if (!empty_list) {
+                const uint32_t col = tq + (uint32_t)(buf * SIDES * Q_BW + side * Q_BW + 8 * j);
+                tmem_ld_32x32b_x8(col, lo);
+                tmem_ld_32x32b_x8(col + Q_BSLOTS, hi);
+                tmem_wait_ld();
+            }
+        };
+        if (half) {  // LB: the sample slots Q_UB_N .. Q_UB_N + Q_LB_N - 1 (chunks 3 .. 7)
+            double lb[SIDES];
+#pragma unroll
+            for (int side = 0; side < SIDES; ++side) {
+                lb[side] = -INFINITY;
+#pragma unroll
+                for (int j = Q_UB_N / 8; j < (Q_UB_N + Q_LB_N + 7) / 8; ++j) {
+                    uint32_t lo[8], hi[8];
+                    load8(side, j, lo, hi);
+#pragma unroll
+                    for (int i = 0; i < 8; ++i) {
+                        const int slot = 8 * j + i;
+                        if (slot < Q_UB_N || slot >= Q_UB_N + Q_LB_N) continue;
+                        const int k = Q_LB_STEP * (slot - Q_UB_N) + Q_LB_OFF;
+                        if (k >= klo[side] && k <= khi[side])
+                            lb[side] = fmax(lb[side], zr[side][slot] + ((double)(int32_t)lo[i] + 256.0 * (int32_t)hi[i]) * (1.0 / 32.0));
+                    }
+                }
+            }
+            tc_fence_before_sync();
+            mbar_arrive(&sm.acc_empty[buf]);
+            if (n_done > 0 && !bound_wait(sm, &sm.lb_empty, (n_done - 1) & 1u)) return;  // half 0 has read the previous LB
+#pragma unroll
+            for (int side = 0; side < SIDES; ++side) sm.lb[side][boot] = lb[side];
+            mbar_arrive(&sm.lb_full);
+        } else {  // UB: the block slots 0 .. Q_UB_N - 1 (chunks 0 .. 3)
+            double ub[SIDES][4];
+#pragma unroll
+            for (int side = 0; side < SIDES; ++side) {
+#pragma unroll
+                for (int pc = 0; pc < 4; ++pc) ub[side][pc] = -INFINITY;
+#pragma unroll
+                for (int j = 0; j < (Q_UB_N + 7) / 8; ++j) {
+                    uint32_t lo[8], hi[8];
+                    load8(side, j, lo, hi);
+#pragma unroll
+                    for (int i = 0; i < 8; ++i) {
+                        const int u = 8 * j + i;
+                        if (u >= Q_UB_N) continue;
+                        const int bl = max(u * Q_UB_PTS, klo[side]), bh = min(u * Q_UB_PTS + Q_UB_PTS - 1, khi[side]);
+                        if (bl > bh) continue;
+                        const double v = zr[side][u] + ((double)(int32_t)lo[i] + 256.0 * (int32_t)hi[i]) * (1.0 / 32.0);
+#pragma unroll
+                        for (int pc = 0; pc < 4; ++pc)
+                            if (max(bl, pc * Q_PW) <= min(bh, pc * Q_PW + Q_PW - 1)) ub[side][pc] = fmax(ub[side][pc], v);
+                    }
+                }
+            }
+            tc_fence_before_sync();
+            mbar_arrive(&sm.acc_empty[buf]);
+            if (!bound_wait(sm, &sm.lb_full, n_done & 1u)) return;
+            double lb[SIDES];
+#pragma unroll
+            for (int side = 0; side < SIDES; ++side) lb[side] = sm.lb[side][boot];
+            mbar_arrive(&sm.lb_empty);
+            uint32_t dead = all;
+#pragma unroll
+            for (int side = 0; side < SIDES; ++side) {
+                if (boot >= p.n_boot[side]) continue;  // a ragged pass: boots past its own count are not real
+                if (side == 0 && p.lb_out) {           // scde_b200_probe_prune_i8
+                    p.lb_out[(int64_t)pos * WP_TILED + boot] = lb[0];
+                    for (int pc = 0; pc < 4; ++pc) p.ub_out[((int64_t)pos * WP_TILED + boot) * 4 + pc] = ub[0][pc];
+                }
+                const double thr = lb[side] - 747.0;  // lb = -inf (no sample inside the range): nothing is dead
+                uint32_t d = 0u;
+#pragma unroll
+                for (int pc = 0; pc < 4; ++pc) d |= ub[side][pc] < thr ? 1u << pc : 0u;
+                dead &= d;
+            }
+            dead = __reduce_and_sync(0xffffffffu, dead);
+            const uint32_t lv = ~dead & all;
+            if (lane == 0 && lv) atomicOr(p.live + (pos >> 2), lv << (8 * (pos & 3)));
+        }
+    }
+}
+
+template <int SIDES>
+__global__ void __launch_bounds__(q_threads(1), 1) bound_i8_kernel(const BoundParams p, int32_t *err) {
+    using G = BoundGeom<SIDES>;
+    constexpr int PRODUCER_WARPS = 4;
+    extern __shared__ __align__(1024) unsigned char smem_raw[];
+    const uint32_t raw = smem_u32(smem_raw);
+    const uint32_t stage0 = (raw + 1023u) & ~1023u;
+    BoundSmem<SIDES> &sm = *reinterpret_cast<BoundSmem<SIDES> *>(smem_raw + (stage0 - raw) + B_RING);
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    if (threadIdx.x == 0) {
+        for (int s = 0; s < G::NS; ++s) {
+            mbar_init(&sm.full[s], 4 * 32);  // one cp.async completion arrival per producer thread
+            mbar_init(&sm.empty[s], 1);      // one tcgen05.commit
+        }
+        for (int b = 0; b < G::NACC; ++b) {
+            mbar_init(&sm.acc_full[b], 1);
+            mbar_init(&sm.acc_empty[b], Q_EPILOGUE_WARPS * 32);
+        }
+        mbar_init(&sm.lb_full, Q_EPILOGUE_WARPS / 2 * 32);
+        mbar_init(&sm.lb_empty, Q_EPILOGUE_WARPS / 2 * 32);
+        sm.abort = 0;
+        mbar_fence_init();
+    }
+    if (warp == PRODUCER_WARPS + Q_EPILOGUE_WARPS) tmem_alloc(&sm.tmem_base, Q_TMEM_COLS);
+    tc_fence_before_sync();
+    __syncthreads();
+    tc_fence_after_sync();
+    const uint32_t tmem = sm.tmem_base;
+    if (warp < PRODUCER_WARPS)
+        bound_producer<SIDES>(p, sm, stage0, warp, lane);
+    else if (warp < PRODUCER_WARPS + Q_EPILOGUE_WARPS)
+        bound_epilogue<SIDES>(p, sm, tmem, warp - PRODUCER_WARPS, lane);  // warp % 4 = its tensor-memory quarter
+    else if (lane == 0)
+        bound_mma<SIDES>(p, sm, stage0, tmem);
+    tc_fence_before_sync();
+    __syncthreads();
+    tc_fence_after_sync();
+    if (sm.abort && err && threadIdx.x == 0) atomicExch(err, 2);
+    if (warp == PRODUCER_WARPS + Q_EPILOGUE_WARPS) tmem_dealloc(tmem, Q_TMEM_COLS);
 }
 
 // items[0 .. *n_live) = the live items' codes in launch order (piece-major or gene-major, as decode_item reads them); one
@@ -1046,11 +1280,11 @@ cudaError_t launch_contract_i8_pass(const ContractI8Args &a, int g0, int n_pos, 
         kernel<<<grid, q_threads(PG), smem, st>>>(p);
         return cudaGetLastError();
     };
-    if (a.hot_rank >= 0) return launch(contract_i8_kernel<PG, true, Q_NS, false>, Q_NS);
+    if (a.hot_rank >= 0) return launch(contract_i8_kernel<PG, true, Q_NS>, Q_NS);
     // the shallow ring leaves 69 KB of shared memory and a third of the register file to a co-resident kernel
-    if (a.ring_stages == 7) return launch(contract_i8_kernel<PG, false, 7, false>, 7);
-    if (a.ring_stages == 8) return launch(contract_i8_kernel<PG, false, 8, false>, 8);
-    return launch(contract_i8_kernel<PG, false, Q_NS, false>, Q_NS);
+    if (a.ring_stages == 7) return launch(contract_i8_kernel<PG, false, 7>, 7);
+    if (a.ring_stages == 8) return launch(contract_i8_kernel<PG, false, 8>, 8);
+    return launch(contract_i8_kernel<PG, false, Q_NS>, Q_NS);
 }
 
 size_t prune_zb_doubles(int n_sets, int n_boot) {
@@ -1064,52 +1298,51 @@ cudaError_t launch_z_bounds(const ContractI8Args &a, const double *Z, int n_sets
     return cudaGetLastError();
 }
 
-size_t prune_bound_ints(int n_pos) { return (size_t)(n_pos > 0 ? n_pos : 1) * WP_TILED * Q_BW; }
-
-cudaError_t launch_bound_pass(const ContractI8Args &a, int g0, int n_pos, const I8Side *s, int n_sides, int n_sm,
-                              cudaStream_t st) {
-    if (n_pos <= 0) return cudaSuccess;
-    if (!a.qbound) return cudaErrorInvalidValue;
-    constexpr int PG = 1;
-    I8Params p = make_params(a, g0, n_pos, s, n_sides);
-    p.qtable = a.qbound;
-    p.ldq = Q_BW;
-    p.n_pieces = 1;
-    p.piece_major = 0;
-    p.items = nullptr;
-    p.n_live = nullptr;
-    // the BOUND kernel stores its int32 sums through T / Tb
-    p.T = reinterpret_cast<long long *>(s[0].S);
-    p.Tb = n_sides > 1 ? reinterpret_cast<long long *>(s[1].S) : nullptr;
-    const int n_items = n_pos << p.twin;
-    int grid = n_sm < n_items ? n_sm : n_items;
-    if (p.twin) grid &= ~1;
-    auto kernel = contract_i8_kernel<PG, false, Q_NS, true>;
-    const size_t smem = q_smem_bytes(Q_NS);
-    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    kernel<<<grid, q_threads(PG), smem, st>>>(p);
-    return cudaGetLastError();
-}
-
-cudaError_t launch_prune_items(const ContractI8Args &a, int g0, int n_pos, const I8Side *s, int n_sides, uint8_t *live,
+cudaError_t launch_prune_items(const ContractI8Args &a, int g0, int n_pos, const I8Side *s, int n_sides, int n_sm, uint8_t *live,
                                int32_t *items, int32_t *n_live, unsigned long long *stats, cudaStream_t st,
                                double *lb_out, double *ub_out) {
     if (n_pos <= 0) return cudaSuccess;
-    const int32_t *order = a.lists.order ? a.lists.order + g0 : nullptr;
-    auto dev = [&](const I8Side &x) {
-        return PruneSideDev{a.row_range ? x.SR : nullptr, x.S, x.zb + (size_t)x.pass * WP_TILED * Q_BSLOTS, side_boots(a, x)};
-    };
-    const int64_t set_zb = (int64_t)prune_zb_doubles(1, a.n_boot);
-    prune_decide_kernel<<<(unsigned)((n_pos + 7) / 8), 256, 0, st>>>(dev(s[0]), dev(s[n_sides - 1]), n_sides, order,
-                                                                     a.gene_set, set_zb, n_pos, a.K, q_pieces(a.K), live,
-                                                                     lb_out, ub_out);
-    cudaError_t e = cudaGetLastError();
+    if (!a.qbound || n_sides < 1 || n_sides > 2) return cudaErrorInvalidValue;
+    BoundParams p{};
+    p.qbound = a.qbound;
+    p.lst_row = a.lists.row;
+    p.lst_cell = a.lists.cell;
+    p.lst_len = a.lists.len;
+    p.order = a.lists.order ? a.lists.order + g0 : nullptr;
+    p.ld_lst = a.lists.ld;
+    p.gene_set = a.gene_set;
+    p.set_w8 = a.set_w8;
+    p.set_zb = (int64_t)prune_zb_doubles(1, a.n_boot);
+    for (int i = 0; i < n_sides; ++i) {
+        p.W8[i] = s[i].W8;
+        p.SR[i] = a.row_range ? s[i].SR : nullptr;
+        p.zb[i] = s[i].zb + (size_t)s[i].pass * WP_TILED * Q_BSLOTS;
+        p.n_boot[i] = side_boots(a, s[i]);
+    }
+    p.n_pos = n_pos;
+    p.K = a.K;
+    p.n_pieces = q_pieces(a.K);
+    p.live = reinterpret_cast<uint32_t *>(live);
+    p.lb_out = lb_out;
+    p.ub_out = ub_out;
+    cudaError_t e = cudaMemsetAsync(live, 0, prune_live_bytes(n_pos), st);
     if (e != cudaSuccess) return e;
-    prune_compact_kernel<<<1, PC_THREADS, 0, st>>>(live, n_pos, q_pieces(a.K), a.item_order == 1, order, a.lists.len, items,
+    const int grid = n_sm < n_pos ? n_sm : n_pos;
+    // function attributes are per device: set on every launch
+    auto launch = [&](auto kernel, size_t smem) -> cudaError_t {
+        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+        kernel<<<grid, q_threads(1), smem, st>>>(p, a.err);
+        return cudaGetLastError();
+    };
+    e = n_sides > 1 ? launch(bound_i8_kernel<2>, bound_smem_bytes<2>()) : launch(bound_i8_kernel<1>, bound_smem_bytes<1>());
+    if (e != cudaSuccess) return e;
+    prune_compact_kernel<<<1, PC_THREADS, 0, st>>>(live, n_pos, q_pieces(a.K), a.item_order == 1, p.order, a.lists.len, items,
                                                    n_live, stats);
     return cudaGetLastError();
 }
+
+size_t prune_live_bytes(int n_pos) { return (size_t)((n_pos > 0 ? n_pos : 1) + 3) & ~(size_t)3; }
 
 cudaError_t launch_exp_probe(double *out_host, cudaStream_t st) {
     double *d = nullptr;
