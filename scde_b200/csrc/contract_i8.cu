@@ -20,17 +20,18 @@
 // reference's soft-max would compare multiples of the sentinel -- and irregular rows raise flag 4: the caller reruns on
 // the FP64 kernel, which adds the sentinels as the reference does.
 //
-// Kernel: persistent, one CTA per SM, three warp roles, no CTA-wide barrier in the steady state.
+// Kernel: persistent, one CTA per SM, three warp roles, no CTA-wide barrier in the steady state (the pipeline skeleton
+// below, which bound_i8_kernel shares).
 //   * work item = (gene, piece): one 512-byte piece of the gene's table rows = 102 grid points x 5 planes.  The item
 //     accumulates D[boot (128 lanes, 104 real)][plane * 102 + i] in all 512 tensor-memory columns of the SM.
-//   * producers (Q_PGROUPS x 4 warps; Q_PGROUPS = 1, see launch_contract_i8_pass): gather the list entries' pieces (512 contiguous, 512-byte-aligned bytes per
-//     entry) and W rows (128 bytes) with 16-byte cp.async straight into the canonical 128-byte-swizzle layout of an
-//     MN-major operand; completion is signalled by cp.async.mbarrier.arrive; a 10-stage ring of 32 entries (20 KB per
-//     stage) keeps up to 200 KB in flight per SM.  The loop is branch-free per stage: constant offsets, slot / phase
-//     counters instead of divisions, list entries fetched 8-16 of the group's stages ahead.
+//   * producers (4 warps): gather the list entries' pieces (512 contiguous, 512-byte-aligned bytes per entry) and W rows
+//     (128 bytes) with 16-byte cp.async straight into the canonical 128-byte-swizzle layout of an MN-major operand;
+//     completion is signalled by cp.async.mbarrier.arrive; a 10-stage ring of 32 entries (20 KB per stage) keeps up to
+//     200 KB in flight per SM.  The loop is branch-free per stage: constant offsets, slot / phase counters instead of
+//     divisions, list entries fetched 8-16 stages ahead.
 //   * MMA (1 thread): per stage two tcgen05.mma (M = 128 boots, N = 256, K = 32 entries), then tcgen05.commit onto the
 //     stage's "empty" barrier; after the last stage a commit onto the accumulator barrier.
-//   * epilogue (4 warps, one per 32-lane quarter of tensor memory): tcgen05.ld the five planes of 8 grid points at a
+//   * epilogue (8 warps, two per 32-lane quarter of tensor memory): tcgen05.ld the five planes of 8 grid points at a
 //     time, recombine into one 64-bit integer per (boot, grid point) and store it; softmax_i8_warp_kernel finishes the gene
 //     (conversion, zero-count base Z[b, k], sentinel ranges, soft-max, average).  Producers keep prefetching the next
 //     item meanwhile.
@@ -53,66 +54,295 @@ constexpr int Q_NS = 10;                         // ring depth (largest; the ker
 constexpr int Q_A_BYTES = Q_ES * Q_WB;           // W tile of a stage: 4096
 constexpr int Q_B_BYTES = Q_ES * Q_PIECE;        // table tile of a stage: 16384
 constexpr int Q_STAGE_BYTES = Q_A_BYTES + Q_B_BYTES;  // 20480, a multiple of the 1024-byte swizzle atom
-// PG producer warp groups (template parameter of the kernel); group g gathers the stages s = g (mod PG) of an item.
+// Warp roles of both tcgen05 kernels: the producer warps, the epilogue warps, then the MMA warp, which also allocates the
+// tensor memory.  ONE producer group: every producer warp touches every stage, so the ring itself bounds the producers'
+// lead.  (Two groups taking alternate stages were no faster and deadlocked: a group with no stage of its own in a run of
+// short items ran ahead until a parity wait on "empty" was satisfied by a phase two uses back -- DESIGN.md 4.3.)
 // Eight epilogue warps: a warp may only read the tensor-memory lanes 32 (warp id mod 4) .. + 31, so two warps share each
-// quarter and split its columns.  (With four warps the epilogue of an item took longer than the ring can cover, and the
-// tensor memory is not free for the next item before it ends.)
+// quarter.  (With four warps the contraction's epilogue of an item took longer than the ring can cover, and the tensor
+// memory is not free for the next item before it ends.)
+constexpr int Q_PRODUCER_WARPS = 4;              // one per 8-entry k-group of a stage
 constexpr int Q_EPILOGUE_WARPS = 8;
-constexpr int q_threads(int pg) { return (4 * pg + Q_EPILOGUE_WARPS + 1) * 32; }  // + the MMA warp
+constexpr int Q_MMA_WARP = Q_PRODUCER_WARPS + Q_EPILOGUE_WARPS;
+constexpr int Q_THREADS = (Q_MMA_WARP + 1) * 32;
 constexpr int Q_EPI_ROUNDS = (Q_PW + 7) / 8;  // rounds of 8 grid points per piece
 constexpr int Q_TMEM_COLS = 512;
 constexpr long long Q_WATCHDOG_CYCLES = 4000000000ll;  // a barrier wait longer than ~2 s aborts the kernel (err = 2)
 static_assert(Q_NV * Q_PW <= Q_TMEM_COLS && Q_NV * Q_PW <= Q_PIECE, "a piece is one pass of tensor memory");
 static_assert((Q_PW & 1) == 0, "the epilogue reads pairs of columns");
 
-struct I8Smem {
-    uint64_t full[Q_NS];
-    uint64_t empty[Q_NS];
-    uint64_t acc_full, acc_empty;
+// The gene lists of a launch and the draw set of every gene, as both tcgen05 kernels read them
+struct ListParams {
+    const int32_t *row, *cell, *len, *order;  // GeneLists, order from the launch's first gene
+    int64_t ld;
+    const int32_t *gene_set;  // draw set of every gene (NULL: one set): its W rows start gene_set[gene] * set_w8 bytes
+    int64_t set_w8;           // after each side's W8
+};
+
+// ---- the pipeline skeleton of both tcgen05 kernels --------------------------------------------------------------------
+// The producer warps gather the Q_ES list entries of a stage into a ring slot with cp.async and arrive on the slot's
+// "full" barrier.  The MMA thread waits on "full", issues the stage's MMAs into the item's accumulator buffer and commits
+// onto the slot's "empty" barrier; after the item's last stage it commits onto the buffer's "full" barrier (or arrives on
+// it: an empty list), and the epilogue warps read the buffer and arrive on its "empty" barrier.  Waiting for the n-th
+// completion (n >= 1) of a barrier is a wait on parity (n - 1) & 1.
+template <int NSB, int NACC>  // NSB >= the ring depth
+struct PipeBars {
+    uint64_t full[NSB], empty[NSB];
+    uint64_t acc_full[NACC], acc_empty[NACC];
     uint32_t tmem_base;
     volatile int abort;
-};
-constexpr int Q_XBUF_BYTES = Q_EPILOGUE_WARPS * 2048;  // per epilogue warp: one [32 boots][8 grid points] tile of 64-bit sums
-constexpr size_t q_smem_bytes(int ns) { return 1024 /* alignment slack */ + (size_t)ns * Q_STAGE_BYTES + Q_XBUF_BYTES + sizeof(I8Smem); }
-
-struct I8Params {
-    const int8_t *qtable;  // [rows][ldq]: row = [piece][plane][102] (+ 2)
-    int64_t ldq;
-    const int32_t *lst_row, *lst_cell, *lst_len, *order;
-    int64_t ld_lst;
-    const int8_t *W8;    // this pass: [n_w_rows][128]
-    const int32_t *gene_set;  // draw set of every gene (NULL: one set): its W rows start gene_set[gene] * set_w8 bytes
-    int64_t set_w8;           // after W8 (and W8b)
-    long long *T;        // [n_pos][104][416]: 2^29 * T[boot, grid] as exact integers (without Z, without sentinels)
-    int n_boot;          // real boots of this pass: rows beyond are not stored
-    int n_pos;           // genes in this launch: positions [0, n_pos) of `order`
-    int n_pieces;        // pieces per gene
-    int32_t *err;        // device flag: 2 = watchdog abort
-    unsigned long long *dbg;  // optional diagnostics: [0] += cycles between "accumulators ready" and "tensor memory released",
-                              // [1] += items, [2] += cycles the MMA thread waited for the release (epilogue warp 0 / MMA thread)
-    const int8_t *W8b;   // twin launch: the second joint's W (same cells, same lists, other draws), else NULL
-    long long *Tb;       // twin launch: the second joint's T tiles
-    int twin;            // 1: items come in pairs (2 i, 2 i + 1) = the same (gene, piece) for joint 0 and joint 1, so that two
-                         // neighbouring CTAs gather the same table rows at the same time and the second read is an L2 hit
-    int piece_major;     // item order: 0 = (gene, piece) with the piece fastest, 1 = (piece, gene) with the gene fastest
-    int cold_evict_first;  // HINT kernels: rows without the hot bit are loaded evict_first (else without a hint)
-    const int32_t *items;  // pruned launch: the codes (item numbers of the order above) of the live items, *n_live of
-    const int32_t *n_live; // them, written on the device by prune_compact_kernel; NULL = every item
+    __device__ __forceinline__ void init(int ns) {  // thread 0, before the init fence
+        for (int s = 0; s < ns; ++s) {
+            mbar_init(&full[s], Q_PRODUCER_WARPS * 32);  // one cp.async completion arrival per producer thread
+            mbar_init(&empty[s], 1);                     // one tcgen05.commit
+        }
+        for (int b = 0; b < NACC; ++b) {
+            mbar_init(&acc_full[b], 1);
+            mbar_init(&acc_empty[b], Q_EPILOGUE_WARPS * 32);
+        }
+        abort = 0;
+    }
 };
 
-template <class Smem>
-__device__ __forceinline__ bool wait_or_abort(Smem &sm, uint64_t *bar, uint32_t parity) {
+// the producer and MMA roles wait spinning; false when the kernel aborts
+__device__ __forceinline__ bool wait_spin(volatile int &abort, uint64_t *bar, uint32_t parity) {
     if (mbar_try_wait(bar, parity)) return true;
     const long long t0 = clock64();
     while (!mbar_try_wait(bar, parity)) {
-        if (sm.abort) return false;
+        if (abort) return false;
         if (clock64() - t0 > Q_WATCHDOG_CYCLES) {  // never in a correct run: leave instead of hanging the GPU
-            sm.abort = 1;
+            abort = 1;
             return false;
         }
     }
     return true;
 }
+// the epilogues' wait: an item takes microseconds, so sleep between polls; false when the kernel aborts
+template <int SLEEP_NS>
+__device__ __forceinline__ bool wait_sleep(volatile int &abort, uint64_t *bar, uint32_t parity) {
+    while (!mbar_try_wait(bar, parity)) {
+        __nanosleep(SLEEP_NS);
+        if (abort) return false;
+    }
+    return true;
+}
+
+// A role's position in the ring of NS stages of STAGE bytes: the slot, and how often it has been filled before.  The
+// producers' and the MMA thread's cursors run across items and visit the same slots in the same order.
+template <int NS, int STAGE>
+struct Ring {
+    uint32_t stage0;
+    int slot = 0;
+    uint32_t fill = 0;
+    __device__ __forceinline__ uint32_t stage() const { return stage0 + (uint32_t)slot * STAGE; }
+    __device__ __forceinline__ void advance() {
+        if (++slot == NS) {
+            slot = 0;
+            ++fill;
+        }
+    }
+};
+
+// The CTA's items blockIdx.x, + gridDim.x, .. < n_items.  gene_of(item) = the item's gene; its list length and (W_SET)
+// the byte offset of its draw set's W rows are loaded one item ahead.  body(item, gene, stages, wset) returns false to
+// stop (abort).
+template <bool W_SET, class GeneOf, class Body>
+__device__ __forceinline__ void walk_items(const ListParams &l, int n_items, GeneOf gene_of, Body body) {
+    int64_t gene_n = 0, wset_n = 0;
+    int len_n = 0;
+    auto fetch = [&](int item) {
+        gene_n = gene_of(item);
+        len_n = l.len[gene_n];
+        if (W_SET && l.gene_set) wset_n = l.gene_set[gene_n] * l.set_w8;
+    };
+    int item = blockIdx.x;
+    if (item < n_items) fetch(item);
+    for (; item < n_items; item += gridDim.x) {
+        const int64_t gene = gene_n, wset = wset_n;
+        const int nst = (len_n + Q_ES - 1) / Q_ES;
+        if (item + (int)gridDim.x < n_items) fetch(item + gridDim.x);
+        if (!body(item, gene, nst, wset)) return;
+    }
+}
+
+template <int DOFF, int SOFF>
+__device__ __forceinline__ void cp_async16_at(uint32_t dst_smem, const void *src) {
+    asm volatile("cp.async.cg.shared.global [%0+%2], [%1+%3], 16;" ::"r"(dst_smem), "l"(src), "n"(DOFF), "n"(SOFF) : "memory");
+}
+template <int DOFF, int SOFF>
+__device__ __forceinline__ void cp_async16_hint_at(uint32_t dst_smem, const void *src, uint64_t policy) {
+    asm volatile("cp.async.cg.shared.global.L2::cache_hint [%0+%2], [%1+%3], 16, %4;" ::"r"(dst_smem), "l"(src), "n"(DOFF), "n"(SOFF),
+                 "l"(policy)
+                 : "memory");
+}
+
+// ---- producers: warp kg gathers entries 8 kg .. 8 kg + 7 (one k-group of the MMA) of every stage ----------------------
+// Canonical 128-byte-swizzle layout of an MN-major operand: the bytes of one entry are split into runs of 128 (8 pieces
+// of 16 bytes); run r of entry kk of k-group kg sits at [r][kg][kk][128 B] and its piece j at 16 * (j ^ kk).  Lane
+// (l3 = lane >> 3, l7 = lane & 7) copies piece l7 of every run of entries l3 and l3 + 4: a warp instruction moves four
+// 128-byte runs of global memory into four 128-byte lines of shared memory -- coalesced on both sides, no bank conflicts.
+//
+// List entries: lane (l3, l7) holds entries l3 and l3 + 4 of the warp's stage 8 t + l7 -- one load instruction fetches
+// the entries of eight stages, issued one block (8 stages) before its first use, the first two blocks at the start of the
+// item; the identity of the NEXT item (gene, list length) is loaded one item ahead.  An earlier version with a shorter
+// look-ahead spent 17 % of the producers' cycles waiting on these loads and 55 % issuing ~180 dependent instructions per
+// stage (profiles/r01v); this loop issues about 45.
+//
+// copy(dst0, dst1, row0, row1, cell0, cell1) issues the cp.async of one stage for this lane's entries l3 and l3 + 4 (their
+// table rows and raw cell words); dst0 / dst1 = their piece l7 in the stage's first 128-byte-swizzled tile.
+template <int NS, int STAGE, int NSB, int NACC, class Copy>
+__device__ __forceinline__ bool gather_item(const ListParams &l, PipeBars<NSB, NACC> &b, Ring<NS, STAGE> &ring, int64_t gene,
+                                            int nst, int kg, int lane, Copy copy) {
+    const int l7 = lane & 7, l3 = lane >> 3;
+    // entry kk = l3 (and l3 + 4): line kk of this warp's k-group, piece l7 at 16 * (l7 ^ kk)
+    const uint32_t d0 = (uint32_t)kg * 1024u + (uint32_t)l3 * 128u + (uint32_t)((l7 ^ l3) << 4);
+    const uint32_t d1 = (uint32_t)kg * 1024u + (uint32_t)(l3 + 4) * 128u + (uint32_t)((l7 ^ (l3 + 4)) << 4);
+    const int32_t *lrow = l.row + gene * l.ld + kg * 8 + l3;
+    const int32_t *lcell = l.cell + gene * l.ld + kg * 8 + l3;
+    int32_t r0a = 0, r1a = 0, c0a = 0, c1a = 0, r0b = 0, r1b = 0, c0b = 0, c1b = 0;
+    auto load_block = [&](int t, int32_t &r0, int32_t &r1, int32_t &c0, int32_t &c1) {
+        const int s = 8 * t + l7;
+        r0 = r1 = c0 = c1 = 0;
+        if (s < nst) {
+            r0 = __ldg(lrow + s * Q_ES);
+            r1 = __ldg(lrow + s * Q_ES + 4);
+            c0 = __ldg(lcell + s * Q_ES);
+            c1 = __ldg(lcell + s * Q_ES + 4);
+        }
+    };
+    load_block(0, r0a, r1a, c0a, c1a);
+    load_block(1, r0b, r1b, c0b, c1b);
+    for (int t = 0; 8 * t < nst; ++t) {
+#pragma unroll
+        for (int u = 0; u < 8; ++u) {
+            if (8 * t + u < nst) {  // warp-uniform
+                const int from = (lane & 24) | u;
+                const int32_t row0 = __shfl_sync(0xffffffffu, r0a, from), row1 = __shfl_sync(0xffffffffu, r1a, from);
+                const int32_t cel0 = __shfl_sync(0xffffffffu, c0a, from), cel1 = __shfl_sync(0xffffffffu, c1a, from);
+                // acquire the slot: the MMAs of its previous fill have read it
+                if (ring.fill > 0 && !wait_spin(b.abort, &b.empty[ring.slot], (ring.fill - 1) & 1u)) return false;
+                const uint32_t sA = ring.stage();
+                copy(sA + d0, sA + d1, row0, row1, cel0, cel1);
+                cp_async_mbar_arrive_noinc(&b.full[ring.slot]);
+                ring.advance();
+            }
+        }
+        r0a = r0b;
+        r1a = r1b;
+        c0a = c0b;
+        c1a = c1b;
+        load_block(t + 2, r0b, r1b, c0b, c1b);
+    }
+    return true;
+}
+
+// The producer role: make_copy(item, wset) returns the copy of one stage of the item (see gather_item)
+template <int NS, int STAGE, int NSB, int NACC, class GeneOf, class MakeCopy>
+__device__ __forceinline__ void run_producer(const ListParams &l, PipeBars<NSB, NACC> &b, uint32_t stage0, int n_items, int kg,
+                                             int lane, GeneOf gene_of, MakeCopy make_copy) {
+    Ring<NS, STAGE> ring{stage0};
+    walk_items<true>(l, n_items, gene_of, [&](int item, int64_t gene, int nst, int64_t wset) {
+        return gather_item(l, b, ring, gene, nst, kg, lane, make_copy(item, wset));
+    });
+}
+
+// The MMA role (one thread): item n goes to accumulator buffer n mod NACC, of Q_TMEM_COLS / NACC columns.
+// issue(stage, acc, accumulate) issues the MMAs of one stage into the buffer at tensor-memory address acc.  dbg (or NULL):
+// [2] += cycles spent waiting for the epilogue to release a buffer.
+template <int NS, int STAGE, int NSB, int NACC, class GeneOf, class Issue>
+__device__ __forceinline__ void run_mma(const ListParams &l, PipeBars<NSB, NACC> &b, uint32_t stage0, uint32_t tmem, int n_items,
+                                        GeneOf gene_of, unsigned long long *dbg, Issue issue) {
+    Ring<NS, STAGE> ring{stage0};
+    uint32_t n_done = 0;
+    walk_items<false>(l, n_items, gene_of, [&](int, int64_t, int nst, int64_t) {
+        const int buf = (int)(n_done % NACC);
+        const uint32_t use = n_done / NACC;
+        ++n_done;
+        if (use > 0) {  // the epilogue has read this buffer's previous item
+            const long long t0 = dbg ? clock64() : 0;
+            if (!wait_spin(b.abort, &b.acc_empty[buf], (use - 1) & 1u)) return false;
+            tc_fence_after_sync();
+            if (dbg) atomicAdd(dbg + 2, (unsigned long long)(clock64() - t0));
+        }
+        const uint32_t acc = tmem + (uint32_t)(buf * (Q_TMEM_COLS / NACC));
+        for (int s = 0; s < nst; ++s) {
+            if (!wait_spin(b.abort, &b.full[ring.slot], ring.fill & 1u)) return false;
+            fence_proxy_async_smem();
+            tc_fence_after_sync();
+            issue(ring.stage(), acc, s > 0);
+            umma_commit(&b.empty[ring.slot]);  // frees the slot once these MMAs have read it
+            ring.advance();
+        }
+        if (nst > 0)
+            umma_commit(&b.acc_full[buf]);
+        else
+            mbar_arrive(&b.acc_full[buf]);  // an empty list: the sums are 0, nothing to wait for
+        return true;
+    });
+}
+
+// The kernel frame: a ring of NS stages from the first 1024-byte boundary of the dynamic shared memory (the swizzle pattern
+// is a function of the shared-memory address bits), the kernel's Smem (whose member `pipe` is its PipeBars) smem_off bytes
+// after the ring's start, all 512 tensor-memory columns, and the three roles: producer(sm, stage0, kg, lane) on the
+// producer warps, epilogue(sm, stage0, tmem, ewarp, lane) on the epilogue warps (ewarp & 3 = the warp's tensor-memory
+// quarter), mma(sm, stage0, tmem) on lane 0 of the MMA warp.  init(sm): thread 0 initialises the kernel's other barriers.
+extern __shared__ __align__(1024) unsigned char q_smem_raw[];
+template <int NS, class Smem, class Init, class Producer, class Epilogue, class Mma>
+__device__ __forceinline__ void run_pipeline(uint32_t smem_off, int32_t *err, Init init, Producer producer, Epilogue epilogue,
+                                             Mma mma) {
+    const uint32_t raw = smem_u32(q_smem_raw);
+    const uint32_t stage0 = (raw + 1023u) & ~1023u;
+    Smem &sm = *reinterpret_cast<Smem *>(q_smem_raw + (stage0 - raw) + smem_off);
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    if (threadIdx.x == 0) {
+        sm.pipe.init(NS);
+        init(sm);
+        mbar_fence_init();
+    }
+    if (warp == Q_MMA_WARP) tmem_alloc(&sm.pipe.tmem_base, Q_TMEM_COLS);
+    tc_fence_before_sync();
+    __syncthreads();
+    tc_fence_after_sync();
+    const uint32_t tmem = sm.pipe.tmem_base;
+    if (warp < Q_PRODUCER_WARPS)
+        producer(sm, stage0, warp, lane);
+    else if (warp < Q_MMA_WARP)
+        epilogue(sm, stage0, tmem, warp - Q_PRODUCER_WARPS, lane);
+    else if (lane == 0)
+        mma(sm, stage0, tmem);
+    tc_fence_before_sync();
+    __syncthreads();
+    tc_fence_after_sync();
+    if (sm.pipe.abort && err && threadIdx.x == 0) atomicExch(err, 2);
+    if (warp == Q_MMA_WARP) tmem_dealloc(tmem, Q_TMEM_COLS);
+}
+
+// ---- contract_i8_kernel -------------------------------------------------------------------------------------------------
+struct I8Smem {
+    PipeBars<Q_NS, 1> pipe;
+};
+constexpr int Q_XBUF_BYTES = Q_EPILOGUE_WARPS * 2048;  // per epilogue warp: one [32 boots][8 grid points] tile of 64-bit sums
+constexpr size_t q_smem_bytes(int ns) { return 1024 /* alignment slack */ + (size_t)ns * Q_STAGE_BYTES + Q_XBUF_BYTES + sizeof(I8Smem); }
+
+struct I8Params {
+    ListParams lists;
+    const int8_t *qtable;  // [rows][ldq]: row = [piece][plane][102] (+ 2)
+    int64_t ldq;
+    const int8_t *W8[2];   // side s: its pass's W rows [n_w_rows][128] (of the first draw set); [1]: twin launches only
+    long long *T[2];       // side s: [n_pos][104][416]: 2^29 * T[boot, grid] as exact integers (without Z, without sentinels)
+    int n_boot;            // real boots of side 0's pass: rows beyond are not stored
+    int n_pos;             // genes in this launch: positions [0, n_pos) of `order`
+    int n_pieces;          // pieces per gene
+    int32_t *err;          // device flag: 2 = watchdog abort
+    unsigned long long *dbg;  // optional diagnostics: [0] += cycles between "accumulators ready" and "tensor memory released",
+                              // [1] += items, [2] += cycles the MMA thread waited for the release (epilogue warp 0 / MMA thread)
+    int twin;            // 1: two sides, items come in pairs (2 i, 2 i + 1) = the same (gene, piece) for side 0 and side 1, so
+                         // that two neighbouring CTAs gather the same table rows at the same time and the second read is an L2 hit
+    int piece_major;     // item order: 0 = (gene, piece) with the piece fastest, 1 = (piece, gene) with the gene fastest
+    int cold_evict_first;  // HINT kernels: rows without the hot bit are loaded evict_first (else without a hint)
+    const int32_t *items;  // pruned launch: the codes (item numbers of the order above) of the live items, *n_live of
+    const int32_t *n_live; // them, written on the device by prune_compact_kernel; NULL = every item
+};
 
 // item -> (gene position, piece).  Gene-major order: the pieces of one gene go to neighbouring CTAs of the same round, so
 // the W rows and list entries they share are L2 hits for three of the four.  Piece-major order: all CTAs work on the same
@@ -123,7 +353,7 @@ struct Item {
     int pos, piece;
 };
 __device__ __forceinline__ int item_code(const I8Params &p, int item) {
-    item >>= p.twin;  // twin launch: bit 0 of the item selects the joint
+    item >>= p.twin;  // twin launch: bit 0 of the item selects the side
     return p.items ? __ldg(p.items + item) : item;
 }
 __device__ __forceinline__ Item decode_item(const I8Params &p, int item) {
@@ -141,37 +371,15 @@ __device__ __forceinline__ Item decode_item(const I8Params &p, int item) {
 __device__ __forceinline__ int64_t item_gene(const I8Params &p, int item) {
     item = item_code(p, item);
     const int pos = p.piece_major ? item % p.n_pos : item / p.n_pieces;
-    return p.order ? p.order[pos] : pos;
+    return p.lists.order ? p.lists.order[pos] : pos;
 }
 
-// ---- producers ------------------------------------------------------------------------------------------------------
-// Warp (grp, kg) gathers entries 8 kg .. 8 kg + 7 (one k-group of the MMA) of the stages s = grp (mod Q_PGROUPS) of
-// every item.  Canonical 128-byte-swizzle layout of an MN-major operand: the bytes of one entry are split into runs of
-// 128 (8 pieces of 16 bytes); run r of entry kk of k-group kg sits at [r][kg][kk][128 B] and its piece j at
-// 16 * (j ^ kk).  Lane (l3 = lane >> 3, l7 = lane & 7) copies piece l7 of every run of entries l3 and l3 + 4: a warp
-// instruction moves four 128-byte runs of global memory into four 128-byte lines of shared memory -- coalesced on both
-// sides, no bank conflicts.
-//
-// List entries: lane (l3, l7) holds entries l3 and l3 + 4 of the warp's own-stage 8 t + l7 -- one load instruction
-// fetches the entries of eight own-stages, issued one block (8 own-stages = 8 Q_PGROUPS stages) before its first use, the
-// first two blocks at the start of the item; the identity of the NEXT item (gene, list length) is loaded one item
-// ahead.  An earlier version with a shorter look-ahead spent 17 % of the producers' cycles waiting on these loads and
-// 55 % issuing ~180 dependent instructions per stage (profiles/r01v); this loop issues about 45.
-template <int DOFF, int SOFF>
-__device__ __forceinline__ void cp_async16_at(uint32_t dst_smem, const void *src) {
-    asm volatile("cp.async.cg.shared.global [%0+%2], [%1+%3], 16;" ::"r"(dst_smem), "l"(src), "n"(DOFF), "n"(SOFF) : "memory");
-}
-template <int DOFF, int SOFF>
-__device__ __forceinline__ void cp_async16_hint_at(uint32_t dst_smem, const void *src, uint64_t policy) {
-    asm volatile("cp.async.cg.shared.global.L2::cache_hint [%0+%2], [%1+%3], 16, %4;" ::"r"(dst_smem), "l"(src), "n"(DOFF), "n"(SOFF),
-                 "l"(policy)
-                 : "memory");
-}
+// A stage: the W tile (Q_A_BYTES), then the table tile of the item's piece, four 128-byte runs per entry.
 // HINT: list entries carry LIST_HOT_BIT in `cell` when the row is one of the first few of its cell (a small count: such a
 // row is shared by thousands of genes); its pieces are loaded with the L2 evict_last policy, the others evict_first (or
 // unhinted), so that the stream of rows that are used once does not push the shared ones out of the L2.
-template <int Q_PGROUPS, bool HINT, int NS>
-__device__ __forceinline__ void run_producer(const I8Params &p, I8Smem &sm, uint32_t stage0, int n_items, int warp, int lane) {
+template <bool HINT, int NS>
+__device__ __forceinline__ void contract_producer(const I8Params &p, I8Smem &sm, uint32_t stage0, int n_items, int kg, int lane) {
     uint64_t pol_hot = 0, pol_cold = 0;
     if (HINT) {
         asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol_hot));
@@ -180,153 +388,44 @@ __device__ __forceinline__ void run_producer(const I8Params &p, I8Smem &sm, uint
         else
             asm volatile("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;" : "=l"(pol_cold));
     }
-    const int grp = warp >> 2, kg = warp & 3;
-    const int l7 = lane & 7, l3 = lane >> 3;
-    // entry kk = l3 (and l3 + 4): line kk of this warp's k-group, piece l7 at 16 * (l7 ^ kk)
-    const uint32_t d0 = (uint32_t)kg * 1024u + (uint32_t)l3 * 128u + (uint32_t)((l7 ^ l3) << 4);
-    const uint32_t d1 = (uint32_t)kg * 1024u + (uint32_t)(l3 + 4) * 128u + (uint32_t)((l7 ^ (l3 + 4)) << 4);
-    int slot_b = 0;        // ring slot of the first stage of the current item
-    uint32_t fill_b = 0;   // how often that slot has been filled before
-    int item = blockIdx.x;
-    int64_t gene_n = 0, wset_n = 0;  // wset: byte offset of the gene's draw set in W8
-    int len_n = 0;
-    if (item < n_items) {
-        gene_n = item_gene(p, item);
-        len_n = p.lst_len[gene_n];
-        if (p.gene_set) wset_n = p.gene_set[gene_n] * p.set_w8;
-    }
-    for (; item < n_items; item += gridDim.x) {
-        const Item it = decode_item(p, item);
-        const int64_t gene = gene_n, wset = wset_n;
-        const int nst = (len_n + Q_ES - 1) / Q_ES;
-        if (item + (int)gridDim.x < n_items) {
-            gene_n = item_gene(p, item + gridDim.x);
-            len_n = p.lst_len[gene_n];
-            if (p.gene_set) wset_n = p.gene_set[gene_n] * p.set_w8;
-        }
-        const int8_t *qbase = p.qtable + (int64_t)it.piece * Q_PIECE + l7 * 16;
-        const int8_t *wbase = ((p.twin && (item & 1)) ? p.W8b : p.W8) + l7 * 16 + wset;
-        const int32_t *lrow = p.lst_row + gene * p.ld_lst + kg * 8 + l3;
-        const int32_t *lcell = p.lst_cell + gene * p.ld_lst + kg * 8 + l3;
-        int32_t r0a = 0, r1a = 0, c0a = 0, c1a = 0, r0b = 0, r1b = 0, c0b = 0, c1b = 0;
-        auto load_block = [&](int t, int32_t &r0, int32_t &r1, int32_t &c0, int32_t &c1) {
-            const int s = grp + Q_PGROUPS * (8 * t + l7);
-            r0 = r1 = c0 = c1 = 0;
-            if (s < nst) {
-                r0 = __ldg(lrow + s * Q_ES);
-                r1 = __ldg(lrow + s * Q_ES + 4);
-                c0 = __ldg(lcell + s * Q_ES);
-                c1 = __ldg(lcell + s * Q_ES + 4);
-            }
-        };
-        load_block(0, r0a, r1a, c0a, c1a);
-        load_block(1, r0b, r1b, c0b, c1b);
-        int slot = slot_b + grp;
-        uint32_t fill = fill_b;
-        if (slot >= NS) {
-            slot -= NS;
-            ++fill;
-        }
-        for (int t = 0; grp + Q_PGROUPS * 8 * t < nst; ++t) {
-#pragma unroll
-            for (int u = 0; u < 8; ++u) {
-                const int s = grp + Q_PGROUPS * (8 * t + u);
-                if (s < nst) {  // warp-uniform
-                    const int from = (lane & 24) | u;
-                    const int32_t row0 = __shfl_sync(0xffffffffu, r0a, from), row1 = __shfl_sync(0xffffffffu, r1a, from);
-                    const int32_t cel0 = __shfl_sync(0xffffffffu, c0a, from), cel1 = __shfl_sync(0xffffffffu, c1a, from);
-                    const uint32_t sA = stage0 + (uint32_t)slot * Q_STAGE_BYTES;
-                    const uint32_t sB0 = sA + Q_A_BYTES + d0, sB1 = sA + Q_A_BYTES + d1;
-                    const int8_t *src0 = qbase + (int64_t)row0 * p.ldq;
-                    const int8_t *src1 = qbase + (int64_t)row1 * p.ldq;
-                    const int8_t *w0 = wbase + (int64_t)(cel0 & ~LIST_HOT_BIT) * Q_WB;
-                    const int8_t *w1 = wbase + (int64_t)(cel1 & ~LIST_HOT_BIT) * Q_WB;
-                    if (fill > 0 && !wait_or_abort(sm, &sm.empty[slot], (fill - 1) & 1u)) return;
-                    if (HINT) {
-                        const uint64_t pol0 = (cel0 & LIST_HOT_BIT) ? pol_hot : pol_cold;
-                        const uint64_t pol1 = (cel1 & LIST_HOT_BIT) ? pol_hot : pol_cold;
-                        cp_async16_hint_at<0, 0>(sB0, src0, pol0);
-                        cp_async16_hint_at<0, 0>(sB1, src1, pol1);
-                        cp_async16_hint_at<4096, 128>(sB0, src0, pol0);
-                        cp_async16_hint_at<4096, 128>(sB1, src1, pol1);
-                        cp_async16_hint_at<8192, 256>(sB0, src0, pol0);
-                        cp_async16_hint_at<8192, 256>(sB1, src1, pol1);
-                        cp_async16_hint_at<12288, 384>(sB0, src0, pol0);
-                        cp_async16_hint_at<12288, 384>(sB1, src1, pol1);
-                        cp_async16_hint_at<0, 0>(sA + d0, w0, pol_hot);
-                        cp_async16_hint_at<0, 0>(sA + d1, w1, pol_hot);
-                    } else {
-                        cp_async16_at<0, 0>(sB0, src0);
-                        cp_async16_at<0, 0>(sB1, src1);
-                        cp_async16_at<4096, 128>(sB0, src0);
-                        cp_async16_at<4096, 128>(sB1, src1);
-                        cp_async16_at<8192, 256>(sB0, src0);
-                        cp_async16_at<8192, 256>(sB1, src1);
-                        cp_async16_at<12288, 384>(sB0, src0);
-                        cp_async16_at<12288, 384>(sB1, src1);
-                        cp_async16_at<0, 0>(sA + d0, w0);
-                        cp_async16_at<0, 0>(sA + d1, w1);
-                    }
-                    cp_async_mbar_arrive_noinc(&sm.full[slot]);
-                    slot += Q_PGROUPS;
-                    if (slot >= NS) {
-                        slot -= NS;
-                        ++fill;
-                    }
+    const int l7 = lane & 7;
+    run_producer<NS, Q_STAGE_BYTES>(
+        p.lists, sm.pipe, stage0, n_items, kg, lane, [&](int item) { return item_gene(p, item); },
+        [&](int item, int64_t wset) {
+            const int8_t *qbase = p.qtable + (int64_t)decode_item(p, item).piece * Q_PIECE + l7 * 16;
+            const int8_t *wbase = ((p.twin && (item & 1)) ? p.W8[1] : p.W8[0]) + l7 * 16 + wset;
+            return [=, &p](uint32_t dst0, uint32_t dst1, int32_t row0, int32_t row1, int32_t cel0, int32_t cel1) {
+                const int8_t *src0 = qbase + (int64_t)row0 * p.ldq;
+                const int8_t *src1 = qbase + (int64_t)row1 * p.ldq;
+                const int8_t *w0 = wbase + (int64_t)(cel0 & ~LIST_HOT_BIT) * Q_WB;
+                const int8_t *w1 = wbase + (int64_t)(cel1 & ~LIST_HOT_BIT) * Q_WB;
+                if (HINT) {
+                    const uint64_t pol0 = (cel0 & LIST_HOT_BIT) ? pol_hot : pol_cold;
+                    const uint64_t pol1 = (cel1 & LIST_HOT_BIT) ? pol_hot : pol_cold;
+                    cp_async16_hint_at<Q_A_BYTES, 0>(dst0, src0, pol0);
+                    cp_async16_hint_at<Q_A_BYTES, 0>(dst1, src1, pol1);
+                    cp_async16_hint_at<Q_A_BYTES + 4096, 128>(dst0, src0, pol0);
+                    cp_async16_hint_at<Q_A_BYTES + 4096, 128>(dst1, src1, pol1);
+                    cp_async16_hint_at<Q_A_BYTES + 8192, 256>(dst0, src0, pol0);
+                    cp_async16_hint_at<Q_A_BYTES + 8192, 256>(dst1, src1, pol1);
+                    cp_async16_hint_at<Q_A_BYTES + 12288, 384>(dst0, src0, pol0);
+                    cp_async16_hint_at<Q_A_BYTES + 12288, 384>(dst1, src1, pol1);
+                    cp_async16_hint_at<0, 0>(dst0, w0, pol_hot);
+                    cp_async16_hint_at<0, 0>(dst1, w1, pol_hot);
+                } else {
+                    cp_async16_at<Q_A_BYTES, 0>(dst0, src0);
+                    cp_async16_at<Q_A_BYTES, 0>(dst1, src1);
+                    cp_async16_at<Q_A_BYTES + 4096, 128>(dst0, src0);
+                    cp_async16_at<Q_A_BYTES + 4096, 128>(dst1, src1);
+                    cp_async16_at<Q_A_BYTES + 8192, 256>(dst0, src0);
+                    cp_async16_at<Q_A_BYTES + 8192, 256>(dst1, src1);
+                    cp_async16_at<Q_A_BYTES + 12288, 384>(dst0, src0);
+                    cp_async16_at<Q_A_BYTES + 12288, 384>(dst1, src1);
+                    cp_async16_at<0, 0>(dst0, w0);
+                    cp_async16_at<0, 0>(dst1, w1);
                 }
-            }
-            r0a = r0b;
-            r1a = r1b;
-            c0a = c0b;
-            c1a = c1b;
-            load_block(t + 2, r0b, r1b, c0b, c1b);
-        }
-        slot_b += nst % NS;
-        fill_b += (uint32_t)(nst / NS);
-        if (slot_b >= NS) {
-            slot_b -= NS;
-            ++fill_b;
-        }
-    }
-}
-
-// ---- MMA issuer (one thread) ------------------------------------------------------------------------------------------
-template <int NS>
-__device__ __forceinline__ void run_mma(const I8Params &p, I8Smem &sm, uint32_t stage0, uint32_t tmem, int n_items) {
-    const uint32_t idesc = umma_idesc_s8_mn(128, 256);
-    int slot = 0;
-    uint32_t fill = 0, n_done = 0;
-    int item = blockIdx.x;
-    int len_n = item < n_items ? p.lst_len[item_gene(p, item)] : 0;
-    for (; item < n_items; item += gridDim.x, ++n_done) {
-        const int nst = (len_n + Q_ES - 1) / Q_ES;
-        if (item + (int)gridDim.x < n_items) len_n = p.lst_len[item_gene(p, item + gridDim.x)];
-        if (n_done > 0) {  // the epilogue has drained the previous item's accumulators
-            const long long t0 = p.dbg ? clock64() : 0;
-            if (!wait_or_abort(sm, &sm.acc_empty, (n_done - 1) & 1u)) return;
-            tc_fence_after_sync();
-            if (p.dbg) atomicAdd(p.dbg + 2, (unsigned long long)(clock64() - t0));
-        }
-        for (int s = 0; s < nst; ++s) {
-            if (!wait_or_abort(sm, &sm.full[slot], fill & 1u)) return;
-            fence_proxy_async_smem();
-            tc_fence_after_sync();
-            const uint32_t sA = stage0 + (uint32_t)slot * Q_STAGE_BYTES;
-            const uint32_t sB = sA + Q_A_BYTES;
-            const uint64_t da = umma_desc_sw128(sA, 4096u, 1024u);
-            umma_s8(tmem, da, umma_desc_sw128(sB, 4096u, 1024u), idesc, s > 0);                      // runs 0, 1
-            umma_s8(tmem + 256u, da, umma_desc_sw128(sB + 2u * 4096u, 4096u, 1024u), idesc, s > 0);  // runs 2, 3
-            umma_commit(&sm.empty[slot]);  // frees the slot once these MMAs have read it
-            if (++slot == NS) {
-                slot = 0;
-                ++fill;
-            }
-        }
-        if (nst > 0)
-            umma_commit(&sm.acc_full);
-        else
-            mbar_arrive(&sm.acc_full);
-    }
+            };
+        });
 }
 
 // ---- epilogue: warps e = 0..7; warp e reads tensor-memory lanes 32 (e & 3) .. + 31 and the rounds of half e >> 2 --------
@@ -337,8 +436,8 @@ __device__ __forceinline__ void run_mma(const I8Params &p, I8Smem &sm, uint32_t 
 // a + 2^16 b + 2^32 s4.  Conversion to FP64, the zero-count base Z and the sentinel ranges are applied by
 // softmax_i8_warp_kernel when it reads T.  (An epilogue that did all of that took 16 800 cycles per item -- 8.9 us, of which
 // the ring hides 3 -- and cost a quarter of the kernel: SCDE_B200_EPI_TIMING, profiles/r01x.)
-__device__ __forceinline__ void run_epilogue(const I8Params &p, I8Smem &sm, uint32_t xbuf, uint32_t tmem, int n_items, int ewarp,
-                                             int lane) {
+__device__ __forceinline__ void contract_epilogue(const I8Params &p, I8Smem &sm, uint32_t xbuf, uint32_t tmem, int n_items,
+                                                  int ewarp, int lane) {
     const int qd = ewarp & 3, half = ewarp >> 2;
     const uint32_t tlane = tmem + ((uint32_t)(qd * 32) << 16);
     // A thread holds 8 grid points of ONE boot (64 bytes of a T row; rows are 3328 bytes apart): stored directly, a warp
@@ -351,15 +450,12 @@ __device__ __forceinline__ void run_epilogue(const I8Params &p, I8Smem &sm, uint
     uint32_t n_done = 0;
     for (int item = blockIdx.x; item < n_items; item += gridDim.x, ++n_done) {
         const Item it = decode_item(p, item);
-        const int64_t gene = p.order ? p.order[it.pos] : it.pos;
-        const bool empty_list = p.lst_len[gene] <= 0;
-        while (!mbar_try_wait(&sm.acc_full, n_done & 1u)) {  // an item takes tens of microseconds: sleep, do not spin
-            __nanosleep(200);
-            if (sm.abort) return;
-        }
+        const int64_t gene = p.lists.order ? p.lists.order[it.pos] : it.pos;
+        const bool empty_list = p.lists.len[gene] <= 0;
+        if (!wait_sleep<200>(sm.pipe.abort, &sm.pipe.acc_full[0], n_done & 1u)) return;
         tc_fence_after_sync();
         const long long t_ready = p.dbg ? clock64() : 0;
-        long long *Tbase = ((p.twin && (item & 1)) ? p.Tb : p.T) + ((int64_t)it.pos * WP_TILED + qd * 32) * KP_TILED + it.piece * Q_PW;
+        long long *Tbase = ((p.twin && (item & 1)) ? p.T[1] : p.T[0]) + ((int64_t)it.pos * WP_TILED + qd * 32) * KP_TILED + it.piece * Q_PW;
         for (int rd = r_begin; rd < r_end; ++rd) {
             const int i0 = rd * 8;
             const int n = Q_PW - i0 < 8 ? Q_PW - i0 : 8;  // 8, or 6 in the last round
@@ -403,7 +499,7 @@ __device__ __forceinline__ void run_epilogue(const I8Params &p, I8Smem &sm, uint
             __syncwarp();
         }
         tc_fence_before_sync();
-        mbar_arrive(&sm.acc_empty);
+        mbar_arrive(&sm.pipe.acc_empty[0]);
         if (p.dbg && ewarp == 0 && lane == 0) {
             atomicAdd(p.dbg, (unsigned long long)(clock64() - t_ready));
             atomicAdd(p.dbg + 1, 1ull);
@@ -411,46 +507,27 @@ __device__ __forceinline__ void run_epilogue(const I8Params &p, I8Smem &sm, uint
     }
 }
 
-template <int Q_PGROUPS, bool HINT, int NS>
-__global__ void __launch_bounds__(q_threads(Q_PGROUPS), 1) contract_i8_kernel(const I8Params p) {
+template <bool HINT, int NS>
+__global__ void __launch_bounds__(Q_THREADS, 1) contract_i8_kernel(const I8Params p) {
     static_assert(NS >= 2 && NS <= Q_NS, "ring depth");
-    constexpr int Q_PRODUCER_WARPS = 4 * Q_PGROUPS;
-    extern __shared__ __align__(1024) unsigned char smem_raw[];
-    // stage buffers on a 1024-byte boundary (the swizzle pattern is a function of the shared-memory address bits)
-    const uint32_t raw = smem_u32(smem_raw);
-    const uint32_t stage0 = (raw + 1023u) & ~1023u;
-    const uint32_t xbuf = stage0 + (uint32_t)NS * Q_STAGE_BYTES;
-    I8Smem &sm = *reinterpret_cast<I8Smem *>(smem_raw + (stage0 - raw) + (size_t)NS * Q_STAGE_BYTES + Q_XBUF_BYTES);
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < NS; ++s) {
-            mbar_init(&sm.full[s], 4 * 32);                 // one cp.async completion arrival per thread of a producer group
-            mbar_init(&sm.empty[s], 1);                     // one tcgen05.commit
-        }
-        mbar_init(&sm.acc_full, 1);
-        mbar_init(&sm.acc_empty, Q_EPILOGUE_WARPS * 32);
-        sm.abort = 0;
-        mbar_fence_init();
-    }
-    if (warp == Q_PRODUCER_WARPS + Q_EPILOGUE_WARPS) tmem_alloc(&sm.tmem_base, Q_TMEM_COLS);
-    tc_fence_before_sync();
-    __syncthreads();
-    tc_fence_after_sync();
-    const uint32_t tmem = sm.tmem_base;
     const int n_items = (p.items ? *p.n_live : p.n_pos * p.n_pieces) << p.twin;
-
-    if (warp < Q_PRODUCER_WARPS)
-        run_producer<Q_PGROUPS, HINT, NS>(p, sm, stage0, n_items, warp, lane);
-    else if (warp < Q_PRODUCER_WARPS + Q_EPILOGUE_WARPS)
-        run_epilogue(p, sm, xbuf, tmem, n_items, warp - Q_PRODUCER_WARPS, lane);
-    else if (lane == 0)
-        run_mma<NS>(p, sm, stage0, tmem, n_items);
-
-    tc_fence_before_sync();
-    __syncthreads();
-    tc_fence_after_sync();
-    if (sm.abort && p.err && threadIdx.x == 0) atomicExch(p.err, 2);
-    if (warp == Q_PRODUCER_WARPS + Q_EPILOGUE_WARPS) tmem_dealloc(tmem, Q_TMEM_COLS);
+    run_pipeline<NS, I8Smem>(
+        NS * Q_STAGE_BYTES + Q_XBUF_BYTES, p.err, [](I8Smem &) {},
+        [&](I8Smem &sm, uint32_t stage0, int kg, int lane) { contract_producer<HINT, NS>(p, sm, stage0, n_items, kg, lane); },
+        [&](I8Smem &sm, uint32_t stage0, uint32_t tmem, int ewarp, int lane) {
+            contract_epilogue(p, sm, stage0 + NS * Q_STAGE_BYTES, tmem, n_items, ewarp, lane);
+        },
+        [&](I8Smem &sm, uint32_t stage0, uint32_t tmem) {
+            const uint32_t idesc = umma_idesc_s8_mn(128, 256);
+            run_mma<NS, Q_STAGE_BYTES>(p.lists, sm.pipe, stage0, tmem, n_items, [&](int item) { return item_gene(p, item); }, p.dbg,
+                                       [&](uint32_t sA, uint32_t acc, bool accumulate) {
+                                           const uint32_t sB = sA + Q_A_BYTES;
+                                           const uint64_t da = umma_desc_sw128(sA, 4096u, 1024u);
+                                           umma_s8(acc, da, umma_desc_sw128(sB, 4096u, 1024u), idesc, accumulate);  // runs 0, 1
+                                           umma_s8(acc + 256u, da, umma_desc_sw128(sB + 2u * 4096u, 4096u, 1024u), idesc,
+                                                   accumulate);  // runs 2, 3
+                                       });
+        });
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -712,15 +789,14 @@ __global__ void z_bounds_kernel(const double *__restrict__ Z, int64_t n_rows, in
 
 // ---- bound_i8_kernel: the bound sums and the decision in one pass -------------------------------------------------------
 // live[pos] = the pieces of gene order[pos] that are not dead for every real boot of the launch's sides.  Persistent, one
-// CTA per SM, item = one gene with both sides of a two-sided launch, the contraction kernel's three warp roles in a
-// geometry of its own:
-//   * producers (4 warps, one group: the ring bounds their lead, see launch_contract_i8_pass): a stage is 32 list
-//     entries -- each side's 128-byte W rows and, gathered ONCE for both sides, the 128-byte bound rows -- copied with
-//     16-byte cp.async into the 128-byte-swizzle layout (the contraction's producer loop).  B_RING = 192 KB of 8 or 12 KB
-//     stages are in flight per SM; the contraction's ring, whose 20 KB stages a bound stage filled only 8 KB of, held 80.
+// CTA per SM, item = one gene with both sides of a two-sided launch, the contraction's pipeline skeleton in a geometry of
+// its own:
+//   * producers: a stage is 32 list entries -- each side's 128-byte W rows and, gathered ONCE for both sides, the
+//     128-byte bound rows.  B_RING = 192 KB of 8 or 12 KB stages are in flight per SM; the contraction's ring, whose
+//     20 KB stages a bound stage filled only 8 KB of, held 80.
 //   * MMA (1 thread): per stage and side one tcgen05.mma (M = 128 boots, N = 128 bound columns, K = 32 entries) into the
-//     side's accumulator of the gene's buffer.  The 512 tensor-memory columns hold 4 buffers (one side) or 2 (two), each
-//     with its own full / empty barrier, so the MMAs of the next genes run while the epilogue reads this one.
+//     side's accumulator of the gene's buffer.  The 512 tensor-memory columns hold 4 buffers (one side) or 2 (two), so
+//     the MMAs of the next genes run while the epilogue reads this one.
 //   * epilogue (8 warps): a thread owns one boot (tensor-memory lane) of its warp's quarter.  The warps of half 1 form LB
 //     from the sample slots, those of half 0 UB_p from the block slots -- both digits of a slot in one thread -- with the
 //     arithmetic of the formulas above; LB reaches the UB thread of its boot through shared memory.  The dead pieces are
@@ -736,22 +812,17 @@ struct BoundGeom {
 };
 template <int SIDES>
 struct BoundSmem {
-    uint64_t full[BoundGeom<SIDES>::NS], empty[BoundGeom<SIDES>::NS];
-    uint64_t acc_full[BoundGeom<SIDES>::NACC], acc_empty[BoundGeom<SIDES>::NACC];
+    PipeBars<BoundGeom<SIDES>::NS, BoundGeom<SIDES>::NACC> pipe;
     uint64_t lb_full, lb_empty;  // the LB exchange: written by half 1, read by half 0
     double lb[SIDES][Q_WB];
-    uint32_t tmem_base;
-    volatile int abort;
 };
 template <int SIDES>
 constexpr size_t bound_smem_bytes() { return 1024 /* alignment slack */ + (size_t)B_RING + sizeof(BoundSmem<SIDES>); }
 
 struct BoundParams {
+    ListParams lists;
     const int8_t *qbound;  // the table's bound rows [rows][Q_BW]
-    const int32_t *lst_row, *lst_cell, *lst_len, *order;
-    int64_t ld_lst;
-    const int32_t *gene_set;  // draw set of every gene (NULL: one set)
-    int64_t set_w8, set_zb;   // bytes of W8 / doubles of zb per draw set
+    int64_t set_zb;           // doubles of zb per draw set
     const int8_t *W8[2];      // side s: its pass's W rows [n_w_rows][128] (of the first draw set)
     const uint32_t *SR[2];    // side s: sentinel ranges [n_pos][128], or NULL (no row holds a sentinel)
     const double *zb[2];      // side s: its pass's Z extrema [104][Q_BSLOTS] (of the first draw set)
@@ -761,130 +832,31 @@ struct BoundParams {
     double *lb_out, *ub_out;  // side 0's LB [n_pos][104] and UB [n_pos][104][4] (scde_b200_probe_prune_i8), or NULL
 };
 
+__device__ __forceinline__ int64_t bound_gene(const BoundParams &p, int pos) { return p.lists.order ? p.lists.order[pos] : pos; }
+
+// A stage: the sides' W tiles, then the bound-row tile
 template <int SIDES>
-__device__ __forceinline__ void bound_producer(const BoundParams &p, BoundSmem<SIDES> &sm, uint32_t stage0, int warp, int lane) {
+__device__ __forceinline__ void bound_producer(const BoundParams &p, BoundSmem<SIDES> &sm, uint32_t stage0, int kg, int lane) {
     using G = BoundGeom<SIDES>;
-    const int kg = warp, l7 = lane & 7, l3 = lane >> 3;
-    const uint32_t d0 = (uint32_t)kg * 1024u + (uint32_t)l3 * 128u + (uint32_t)((l7 ^ l3) << 4);
-    const uint32_t d1 = (uint32_t)kg * 1024u + (uint32_t)(l3 + 4) * 128u + (uint32_t)((l7 ^ (l3 + 4)) << 4);
-    int slot = 0;
-    uint32_t fill = 0;
-    int pos = blockIdx.x;
-    int64_t gene_n = 0, wset_n = 0;
-    int len_n = 0;
-    if (pos < p.n_pos) {
-        gene_n = p.order ? p.order[pos] : pos;
-        len_n = p.lst_len[gene_n];
-        if (p.gene_set) wset_n = p.gene_set[gene_n] * p.set_w8;
-    }
-    for (; pos < p.n_pos; pos += gridDim.x) {
-        const int64_t gene = gene_n, wset = wset_n;
-        const int nst = (len_n + Q_ES - 1) / Q_ES;
-        if (pos + (int)gridDim.x < p.n_pos) {
-            gene_n = p.order ? p.order[pos + gridDim.x] : pos + gridDim.x;
-            len_n = p.lst_len[gene_n];
-            if (p.gene_set) wset_n = p.gene_set[gene_n] * p.set_w8;
-        }
-        const int8_t *qbase = p.qbound + l7 * 16;
-        const int8_t *wb0 = p.W8[0] + wset + l7 * 16;
-        const int8_t *wb1 = p.W8[SIDES - 1] + wset + l7 * 16;
-        const int32_t *lrow = p.lst_row + gene * p.ld_lst + kg * 8 + l3;
-        const int32_t *lcell = p.lst_cell + gene * p.ld_lst + kg * 8 + l3;
-        int32_t r0a = 0, r1a = 0, c0a = 0, c1a = 0, r0b = 0, r1b = 0, c0b = 0, c1b = 0;
-        auto load_block = [&](int t, int32_t &r0, int32_t &r1, int32_t &c0, int32_t &c1) {
-            const int s = 8 * t + l7;
-            r0 = r1 = c0 = c1 = 0;
-            if (s < nst) {
-                r0 = __ldg(lrow + s * Q_ES);
-                r1 = __ldg(lrow + s * Q_ES + 4);
-                c0 = __ldg(lcell + s * Q_ES);
-                c1 = __ldg(lcell + s * Q_ES + 4);
-            }
-        };
-        load_block(0, r0a, r1a, c0a, c1a);
-        load_block(1, r0b, r1b, c0b, c1b);
-        for (int t = 0; 8 * t < nst; ++t) {
-#pragma unroll
-            for (int u = 0; u < 8; ++u) {
-                if (8 * t + u < nst) {  // warp-uniform
-                    const int from = (lane & 24) | u;
-                    const int32_t row0 = __shfl_sync(0xffffffffu, r0a, from), row1 = __shfl_sync(0xffffffffu, r1a, from);
-                    const int64_t cel0 = __shfl_sync(0xffffffffu, c0a, from) & ~LIST_HOT_BIT;
-                    const int64_t cel1 = __shfl_sync(0xffffffffu, c1a, from) & ~LIST_HOT_BIT;
-                    const uint32_t sA = stage0 + (uint32_t)slot * G::STAGE, sB = sA + SIDES * B_TILE;
-                    if (fill > 0 && !wait_or_abort(sm, &sm.empty[slot], (fill - 1) & 1u)) return;
-                    cp_async16_at<0, 0>(sB + d0, qbase + (int64_t)row0 * Q_BW);
-                    cp_async16_at<0, 0>(sB + d1, qbase + (int64_t)row1 * Q_BW);
-                    cp_async16_at<0, 0>(sA + d0, wb0 + cel0 * Q_WB);
-                    cp_async16_at<0, 0>(sA + d1, wb0 + cel1 * Q_WB);
-                    if (SIDES > 1) {
-                        cp_async16_at<B_TILE, 0>(sA + d0, wb1 + cel0 * Q_WB);
-                        cp_async16_at<B_TILE, 0>(sA + d1, wb1 + cel1 * Q_WB);
-                    }
-                    cp_async_mbar_arrive_noinc(&sm.full[slot]);
-                    if (++slot == G::NS) {
-                        slot = 0;
-                        ++fill;
-                    }
+    const int l7 = lane & 7;
+    run_producer<G::NS, G::STAGE>(
+        p.lists, sm.pipe, stage0, p.n_pos, kg, lane, [&](int pos) { return bound_gene(p, pos); },
+        [&](int, int64_t wset) {
+            const int8_t *qbase = p.qbound + l7 * 16;
+            const int8_t *wb0 = p.W8[0] + wset + l7 * 16;
+            const int8_t *wb1 = p.W8[SIDES - 1] + wset + l7 * 16;
+            return [=](uint32_t dst0, uint32_t dst1, int32_t row0, int32_t row1, int32_t cel0, int32_t cel1) {
+                const int64_t c0 = cel0 & ~LIST_HOT_BIT, c1 = cel1 & ~LIST_HOT_BIT;
+                cp_async16_at<SIDES * B_TILE, 0>(dst0, qbase + (int64_t)row0 * Q_BW);
+                cp_async16_at<SIDES * B_TILE, 0>(dst1, qbase + (int64_t)row1 * Q_BW);
+                cp_async16_at<0, 0>(dst0, wb0 + c0 * Q_WB);
+                cp_async16_at<0, 0>(dst1, wb0 + c1 * Q_WB);
+                if (SIDES > 1) {
+                    cp_async16_at<B_TILE, 0>(dst0, wb1 + c0 * Q_WB);
+                    cp_async16_at<B_TILE, 0>(dst1, wb1 + c1 * Q_WB);
                 }
-            }
-            r0a = r0b;
-            r1a = r1b;
-            c0a = c0b;
-            c1a = c1b;
-            load_block(t + 2, r0b, r1b, c0b, c1b);
-        }
-    }
-}
-
-template <int SIDES>
-__device__ __forceinline__ void bound_mma(const BoundParams &p, BoundSmem<SIDES> &sm, uint32_t stage0, uint32_t tmem) {
-    using G = BoundGeom<SIDES>;
-    const uint32_t idesc = umma_idesc_s8_mn(128, Q_BW);
-    int slot = 0;
-    uint32_t fill = 0, n_done = 0;
-    int pos = blockIdx.x;
-    int len_n = pos < p.n_pos ? p.lst_len[p.order ? p.order[pos] : pos] : 0;
-    for (; pos < p.n_pos; pos += gridDim.x, ++n_done) {
-        const int nst = (len_n + Q_ES - 1) / Q_ES;
-        if (pos + (int)gridDim.x < p.n_pos) len_n = p.lst_len[p.order ? p.order[pos + gridDim.x] : pos + gridDim.x];
-        const int buf = (int)(n_done % G::NACC);
-        const uint32_t use = n_done / G::NACC;
-        if (use > 0) {  // the epilogue has read this buffer's previous gene
-            if (!wait_or_abort(sm, &sm.acc_empty[buf], (use - 1) & 1u)) return;
-            tc_fence_after_sync();
-        }
-        const uint32_t acc = tmem + (uint32_t)(buf * SIDES * Q_BW);
-        for (int s = 0; s < nst; ++s) {
-            if (!wait_or_abort(sm, &sm.full[slot], fill & 1u)) return;
-            fence_proxy_async_smem();
-            tc_fence_after_sync();
-            const uint32_t sA = stage0 + (uint32_t)slot * G::STAGE;
-            const uint64_t db = umma_desc_sw128(sA + SIDES * B_TILE, 4096u, 1024u);
-#pragma unroll
-            for (int side = 0; side < SIDES; ++side)
-                umma_s8(acc + (uint32_t)(side * Q_BW), umma_desc_sw128(sA + side * B_TILE, 4096u, 1024u), db, idesc, s > 0);
-            umma_commit(&sm.empty[slot]);
-            if (++slot == G::NS) {
-                slot = 0;
-                ++fill;
-            }
-        }
-        if (nst > 0)
-            umma_commit(&sm.acc_full[buf]);
-        else
-            mbar_arrive(&sm.acc_full[buf]);  // an empty list: the sums are 0, nothing to wait for
-    }
-}
-
-// the epilogue's waits: a gene takes microseconds, so sleep between polls; false when the kernel aborts
-template <int SIDES>
-__device__ __forceinline__ bool bound_wait(BoundSmem<SIDES> &sm, uint64_t *bar, uint32_t parity) {
-    while (!mbar_try_wait(bar, parity)) {
-        __nanosleep(100);
-        if (sm.abort) return false;
-    }
-    return true;
+            };
+        });
 }
 
 template <int SIDES>
@@ -896,9 +868,9 @@ __device__ __forceinline__ void bound_epilogue(const BoundParams &p, BoundSmem<S
     const uint32_t all = (1u << p.n_pieces) - 1u;
     uint32_t n_done = 0;
     for (int pos = blockIdx.x; pos < p.n_pos; pos += gridDim.x, ++n_done) {
-        const int64_t gene = p.order ? p.order[pos] : pos;
-        const bool empty_list = p.lst_len[gene] <= 0;
-        const int64_t zoff = p.gene_set ? p.gene_set[gene] * p.set_zb : 0;
+        const int64_t gene = bound_gene(p, pos);
+        const bool empty_list = p.lists.len[gene] <= 0;
+        const int64_t zoff = p.lists.gene_set ? p.lists.gene_set[gene] * p.set_zb : 0;
         int klo[SIDES], khi[SIDES];
         const double *zr[SIDES];
 #pragma unroll
@@ -909,7 +881,7 @@ __device__ __forceinline__ void bound_epilogue(const BoundParams &p, BoundSmem<S
             zr[side] = p.zb[side] + zoff + (int64_t)(boot < p.n_boot[side] ? boot : 0) * Q_BSLOTS;  // past the boots: not used
         }
         const int buf = (int)(n_done % G::NACC);
-        if (!bound_wait(sm, &sm.acc_full[buf], (n_done / G::NACC) & 1u)) return;
+        if (!wait_sleep<100>(sm.pipe.abort, &sm.pipe.acc_full[buf], (n_done / G::NACC) & 1u)) return;
         tc_fence_after_sync();
         // slot i of the bound row: digits in columns i and Q_BSLOTS + i, read 8 slots at a time
         auto load8 = [&](int side, int j, uint32_t (&lo)[8], uint32_t (&hi)[8]) {
@@ -942,8 +914,9 @@ __device__ __forceinline__ void bound_epilogue(const BoundParams &p, BoundSmem<S
                 }
             }
             tc_fence_before_sync();
-            mbar_arrive(&sm.acc_empty[buf]);
-            if (n_done > 0 && !bound_wait(sm, &sm.lb_empty, (n_done - 1) & 1u)) return;  // half 0 has read the previous LB
+            mbar_arrive(&sm.pipe.acc_empty[buf]);
+            // half 0 has read the previous LB
+            if (n_done > 0 && !wait_sleep<100>(sm.pipe.abort, &sm.lb_empty, (n_done - 1) & 1u)) return;
 #pragma unroll
             for (int side = 0; side < SIDES; ++side) sm.lb[side][boot] = lb[side];
             mbar_arrive(&sm.lb_full);
@@ -971,8 +944,8 @@ __device__ __forceinline__ void bound_epilogue(const BoundParams &p, BoundSmem<S
                 }
             }
             tc_fence_before_sync();
-            mbar_arrive(&sm.acc_empty[buf]);
-            if (!bound_wait(sm, &sm.lb_full, n_done & 1u)) return;
+            mbar_arrive(&sm.pipe.acc_empty[buf]);
+            if (!wait_sleep<100>(sm.pipe.abort, &sm.lb_full, n_done & 1u)) return;
             double lb[SIDES];
 #pragma unroll
             for (int side = 0; side < SIDES; ++side) lb[side] = sm.lb[side][boot];
@@ -999,44 +972,27 @@ __device__ __forceinline__ void bound_epilogue(const BoundParams &p, BoundSmem<S
 }
 
 template <int SIDES>
-__global__ void __launch_bounds__(q_threads(1), 1) bound_i8_kernel(const BoundParams p, int32_t *err) {
+__global__ void __launch_bounds__(Q_THREADS, 1) bound_i8_kernel(const BoundParams p, int32_t *err) {
     using G = BoundGeom<SIDES>;
-    constexpr int PRODUCER_WARPS = 4;
-    extern __shared__ __align__(1024) unsigned char smem_raw[];
-    const uint32_t raw = smem_u32(smem_raw);
-    const uint32_t stage0 = (raw + 1023u) & ~1023u;
-    BoundSmem<SIDES> &sm = *reinterpret_cast<BoundSmem<SIDES> *>(smem_raw + (stage0 - raw) + B_RING);
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < G::NS; ++s) {
-            mbar_init(&sm.full[s], 4 * 32);  // one cp.async completion arrival per producer thread
-            mbar_init(&sm.empty[s], 1);      // one tcgen05.commit
-        }
-        for (int b = 0; b < G::NACC; ++b) {
-            mbar_init(&sm.acc_full[b], 1);
-            mbar_init(&sm.acc_empty[b], Q_EPILOGUE_WARPS * 32);
-        }
-        mbar_init(&sm.lb_full, Q_EPILOGUE_WARPS / 2 * 32);
-        mbar_init(&sm.lb_empty, Q_EPILOGUE_WARPS / 2 * 32);
-        sm.abort = 0;
-        mbar_fence_init();
-    }
-    if (warp == PRODUCER_WARPS + Q_EPILOGUE_WARPS) tmem_alloc(&sm.tmem_base, Q_TMEM_COLS);
-    tc_fence_before_sync();
-    __syncthreads();
-    tc_fence_after_sync();
-    const uint32_t tmem = sm.tmem_base;
-    if (warp < PRODUCER_WARPS)
-        bound_producer<SIDES>(p, sm, stage0, warp, lane);
-    else if (warp < PRODUCER_WARPS + Q_EPILOGUE_WARPS)
-        bound_epilogue<SIDES>(p, sm, tmem, warp - PRODUCER_WARPS, lane);  // warp % 4 = its tensor-memory quarter
-    else if (lane == 0)
-        bound_mma<SIDES>(p, sm, stage0, tmem);
-    tc_fence_before_sync();
-    __syncthreads();
-    tc_fence_after_sync();
-    if (sm.abort && err && threadIdx.x == 0) atomicExch(err, 2);
-    if (warp == PRODUCER_WARPS + Q_EPILOGUE_WARPS) tmem_dealloc(tmem, Q_TMEM_COLS);
+    run_pipeline<G::NS, BoundSmem<SIDES>>(
+        B_RING, err,
+        [](BoundSmem<SIDES> &sm) {
+            mbar_init(&sm.lb_full, Q_EPILOGUE_WARPS / 2 * 32);
+            mbar_init(&sm.lb_empty, Q_EPILOGUE_WARPS / 2 * 32);
+        },
+        [&](BoundSmem<SIDES> &sm, uint32_t stage0, int kg, int lane) { bound_producer<SIDES>(p, sm, stage0, kg, lane); },
+        [&](BoundSmem<SIDES> &sm, uint32_t, uint32_t tmem, int ewarp, int lane) { bound_epilogue<SIDES>(p, sm, tmem, ewarp, lane); },
+        [&](BoundSmem<SIDES> &sm, uint32_t stage0, uint32_t tmem) {
+            const uint32_t idesc = umma_idesc_s8_mn(128, Q_BW);
+            run_mma<G::NS, G::STAGE>(p.lists, sm.pipe, stage0, tmem, p.n_pos, [&](int pos) { return bound_gene(p, pos); }, nullptr,
+                                     [&](uint32_t sA, uint32_t acc, bool accumulate) {
+                                         const uint64_t db = umma_desc_sw128(sA + SIDES * B_TILE, 4096u, 1024u);
+#pragma unroll
+                                         for (int side = 0; side < SIDES; ++side)
+                                             umma_s8(acc + (uint32_t)(side * Q_BW), umma_desc_sw128(sA + side * B_TILE, 4096u, 1024u),
+                                                     db, idesc, accumulate);
+                                     });
+        });
 }
 
 // items[0 .. *n_live) = the live items' codes in launch order (piece-major or gene-major, as decode_item reads them); one
@@ -1218,73 +1174,62 @@ static int side_boots(const ContractI8Args &a, const I8Side &s) {
     return (a.n_boot - s.pass * WP_TILED) < WP_TILED ? (a.n_boot - s.pass * WP_TILED) : WP_TILED;
 }
 
-// the kernel's parameters of a launch over the sides s[0 .. n_sides): their W rows and T tiles, side 0's boots
-static I8Params make_params(const ContractI8Args &a, int g0, int n_pos, const I8Side *s, int n_sides) {
-    I8Params p;
-    p.qtable = a.qtable;
-    p.ldq = a.ldq;
-    p.lst_row = a.lists.row;
-    p.lst_cell = a.lists.cell;
-    p.lst_len = a.lists.len;
-    p.order = a.lists.order ? a.lists.order + g0 : nullptr;
-    p.ld_lst = a.lists.ld;
-    p.W8 = s[0].W8;
-    p.gene_set = a.gene_set;
-    p.set_w8 = a.set_w8;
-    p.T = reinterpret_cast<long long *>(s[0].T);
-    p.n_boot = side_boots(a, s[0]);
-    p.n_pos = n_pos;
-    p.n_pieces = q_pieces(a.K);
-    p.err = a.err;
-    p.dbg = a.dbg;
-    p.W8b = n_sides > 1 ? s[1].W8 : nullptr;
-    p.Tb = n_sides > 1 ? reinterpret_cast<long long *>(s[1].T) : nullptr;
-    p.twin = n_sides > 1 ? 1 : 0;
-    p.piece_major = a.item_order == 1;
-    p.cold_evict_first = a.cold_evict_first;
-    p.items = a.items;
-    p.n_live = a.items ? a.n_live : nullptr;
-    return p;
+// the lists of genes order[g0 ..] and the draw sets, as the kernels of a launch at g0 read them
+static ListParams list_params(const ContractI8Args &a, int g0) {
+    return ListParams{a.lists.row, a.lists.cell,  a.lists.len, a.lists.order ? a.lists.order + g0 : nullptr,
+                      a.lists.ld,  a.gene_set,    a.set_w8};
+}
+
+// one launch of a pipeline kernel, one CTA of Q_THREADS per SM; function attributes are per device: set on every launch
+// (a process may hold contexts on several GPUs)
+template <class... Args>
+static cudaError_t launch_pipeline(void (*kernel)(Args...), int grid, size_t smem, cudaStream_t st, Args... args) {
+    const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    kernel<<<grid, Q_THREADS, smem, st>>>(args...);
+    return cudaGetLastError();
 }
 
 cudaError_t launch_sentinel_ranges(const ContractI8Args &a, int g0, int n_pos, const I8Side &s, cudaStream_t st) {
     if (n_pos <= 0 || !a.row_range) return cudaSuccess;
     if (!s.SR) return cudaErrorInvalidValue;
-    const I8Params p = make_params(a, g0, n_pos, &s, 1);
-    sentinel_range_kernel<<<(unsigned)((n_pos + 7) / 8), 256, 0, st>>>(p.lst_row, p.lst_cell, p.lst_len, p.order, p.ld_lst,
-                                                                       a.row_range, p.W8, a.gene_set, a.set_w8, n_pos, a.K,
-                                                                       p.n_boot, s.SR, a.err);
+    const ListParams l = list_params(a, g0);
+    sentinel_range_kernel<<<(unsigned)((n_pos + 7) / 8), 256, 0, st>>>(l.row, l.cell, l.len, l.order, l.ld, a.row_range, s.W8,
+                                                                       l.gene_set, l.set_w8, n_pos, a.K, side_boots(a, s),
+                                                                       s.SR, a.err);
     return cudaGetLastError();
 }
 
 cudaError_t launch_contract_i8_pass(const ContractI8Args &a, int g0, int n_pos, const I8Side *s, int n_sides, int n_sm,
                                     cudaStream_t st) {
     if (n_pos <= 0) return cudaSuccess;
-    // ONE producer group (four warps, one per k-group of a stage).  Round 1 used two groups that took alternate stages:
-    // no faster (74.37 against 74.34 ms per step at config 4, profiles/r02_experiments.txt) and unsafe -- a group that has
-    // no stage of its own in a run of short items (lists of <= 32 entries) does not wait on anything, runs arbitrarily far
-    // ahead of the MMA thread, and its next parity wait on a slot's "empty" barrier can then be satisfied by a phase two
-    // uses back; with the piece-major item order (short items at the end of every phase, long ones at the start of the
-    // next) that deadlocked scde.posteriors over 40 cells (tests: test_config2_..., test_short_and_long_lists_mixed...).
-    // With one group every producer warp touches every stage, so the ring itself bounds its lead.
-    constexpr int PG = 1;
-    const I8Params p = make_params(a, g0, n_pos, s, n_sides);
+    if (n_sides < 1 || n_sides > 2) return cudaErrorInvalidValue;
+    I8Params p{};
+    p.lists = list_params(a, g0);
+    p.qtable = a.qtable;
+    p.ldq = a.ldq;
+    for (int i = 0; i < n_sides; ++i) {
+        p.W8[i] = s[i].W8;
+        p.T[i] = reinterpret_cast<long long *>(s[i].T);
+    }
+    p.n_boot = side_boots(a, s[0]);
+    p.n_pos = n_pos;
+    p.n_pieces = q_pieces(a.K);
+    p.err = a.err;
+    p.dbg = a.dbg;
+    p.twin = n_sides > 1 ? 1 : 0;
+    p.piece_major = a.item_order == 1;
+    p.cold_evict_first = a.cold_evict_first;
+    p.items = a.items;
+    p.n_live = a.items ? a.n_live : nullptr;
     const int n_items = (n_pos * p.n_pieces) << p.twin;
     int grid = n_sm < n_items ? n_sm : n_items;
-    if (p.twin) grid &= ~1;  // an even stride keeps every CTA on one joint and the pairs (2 i, 2 i + 1) together
-    // function attributes are per device: set on every launch (a process may hold contexts on several GPUs)
-    auto launch = [&](auto kernel, int ns) -> cudaError_t {
-        const size_t smem = q_smem_bytes(ns);
-        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        kernel<<<grid, q_threads(PG), smem, st>>>(p);
-        return cudaGetLastError();
-    };
-    if (a.hot_rank >= 0) return launch(contract_i8_kernel<PG, true, Q_NS>, Q_NS);
+    if (p.twin) grid &= ~1;  // an even stride keeps every CTA on one side and the pairs (2 i, 2 i + 1) together
+    if (a.hot_rank >= 0) return launch_pipeline(contract_i8_kernel<true, Q_NS>, grid, q_smem_bytes(Q_NS), st, p);
     // the shallow ring leaves 69 KB of shared memory and a third of the register file to a co-resident kernel
-    if (a.ring_stages == 7) return launch(contract_i8_kernel<PG, false, 7>, 7);
-    if (a.ring_stages == 8) return launch(contract_i8_kernel<PG, false, 8>, 8);
-    return launch(contract_i8_kernel<PG, false, Q_NS>, Q_NS);
+    if (a.ring_stages == 7) return launch_pipeline(contract_i8_kernel<false, 7>, grid, q_smem_bytes(7), st, p);
+    if (a.ring_stages == 8) return launch_pipeline(contract_i8_kernel<false, 8>, grid, q_smem_bytes(8), st, p);
+    return launch_pipeline(contract_i8_kernel<false, Q_NS>, grid, q_smem_bytes(Q_NS), st, p);
 }
 
 size_t prune_zb_doubles(int n_sets, int n_boot) {
@@ -1304,14 +1249,8 @@ cudaError_t launch_prune_items(const ContractI8Args &a, int g0, int n_pos, const
     if (n_pos <= 0) return cudaSuccess;
     if (!a.qbound || n_sides < 1 || n_sides > 2) return cudaErrorInvalidValue;
     BoundParams p{};
+    p.lists = list_params(a, g0);
     p.qbound = a.qbound;
-    p.lst_row = a.lists.row;
-    p.lst_cell = a.lists.cell;
-    p.lst_len = a.lists.len;
-    p.order = a.lists.order ? a.lists.order + g0 : nullptr;
-    p.ld_lst = a.lists.ld;
-    p.gene_set = a.gene_set;
-    p.set_w8 = a.set_w8;
     p.set_zb = (int64_t)prune_zb_doubles(1, a.n_boot);
     for (int i = 0; i < n_sides; ++i) {
         p.W8[i] = s[i].W8;
@@ -1328,17 +1267,11 @@ cudaError_t launch_prune_items(const ContractI8Args &a, int g0, int n_pos, const
     cudaError_t e = cudaMemsetAsync(live, 0, prune_live_bytes(n_pos), st);
     if (e != cudaSuccess) return e;
     const int grid = n_sm < n_pos ? n_sm : n_pos;
-    // function attributes are per device: set on every launch
-    auto launch = [&](auto kernel, size_t smem) -> cudaError_t {
-        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        kernel<<<grid, q_threads(1), smem, st>>>(p, a.err);
-        return cudaGetLastError();
-    };
-    e = n_sides > 1 ? launch(bound_i8_kernel<2>, bound_smem_bytes<2>()) : launch(bound_i8_kernel<1>, bound_smem_bytes<1>());
+    e = n_sides > 1 ? launch_pipeline(bound_i8_kernel<2>, grid, bound_smem_bytes<2>(), st, p, a.err)
+                    : launch_pipeline(bound_i8_kernel<1>, grid, bound_smem_bytes<1>(), st, p, a.err);
     if (e != cudaSuccess) return e;
-    prune_compact_kernel<<<1, PC_THREADS, 0, st>>>(live, n_pos, q_pieces(a.K), a.item_order == 1, p.order, a.lists.len, items,
-                                                   n_live, stats);
+    prune_compact_kernel<<<1, PC_THREADS, 0, st>>>(live, n_pos, q_pieces(a.K), a.item_order == 1, p.lists.order, a.lists.len,
+                                                   items, n_live, stats);
     return cudaGetLastError();
 }
 
