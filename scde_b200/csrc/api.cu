@@ -158,12 +158,69 @@ struct scde_b200_ctx {
 
 namespace {
 
+// One set of per-cell error models on the device (C x 12, column-major) and what building table rows from it needs
+struct ModelSet {
+    DBuf<double> m;
+    int C = 0, local_theta = 0, sqlogit = 0;
+    bool fast_theta = false;  // every corr.theta finite and > 0, no local-theta fit
+};
+
+// What a call asks of its table
+struct TableRequest {
+    const ModelSet *models;  // one row per cell
+    const double *mag;       // device, the grid's magnitudes
+    int K;
+    int clamp_n;  // the reference's "log 0" sentinel is -DBL_MAX / clamp_n / 1.1
+    bool zero_base = false;    // the zero-base form, where the context's zero_base option allows it
+    bool fixed_point = false;  // fixed-point planes for the tcgen05 contraction
+    bool modes = false;        // row_mode, the argmax of every row: only for return.individual.posterior.modes
+    bool probe = false;        // scde_b200_probe_table*: the zero-base form whatever the option
+    bool bounds = false;       // bound rows whatever the number of cells (scde_b200_probe_table_bounds)
+};
+
+// Pruning (DESIGN.md 4.3) pays where a joint has at least this many cells: measured on one B200 (1000 W), config 3 (1000
+// cells per joint) was 3.0 ms per step slower with it (bound pass and bound rows cost more than the 27 % of the gather they
+// removed), config 4 (5000) 7.7 ms faster.  The bound rows are only written for tables of at least as many cells.
+constexpr int PRUNE_MIN_CELLS = 2500;
+
+// Which kernels build a table and what it holds (DESIGN.md 4.2).  The default is a plain FP64 table.  Rows: lp_rows_kernel,
+// lp_rows_fast_kernel with FP64 rows or with fixed-point planes only, lp_rows_q_kernel (planes only).
+enum class Rows { General, Fast, FastPlanes, Q };
+struct TablePlan {
+    bool zero_base = false;  // rows of non-zero counts hold lp(x) - lp(0) of their cell, the zero-count rows lp(0) itself,
+                             // and the contraction only visits the cells whose count is non-zero (boot_contract.cu)
+    bool fast = false;       // the constant-theta kernels: per-row constants, and the zero-count rows in zero-base form
+    Rows rows = Rows::General;  // the producer of the rows of non-zero counts (of every row outside the zero-base form)
+    bool planes = false;     // the table also exists in fixed point (tcgen05 contraction)
+    bool bounds = false;     // ... with the bound rows of pruning
+    bool modes = false;      // row_mode
+    // the FP64 table holds one row per cell, its zero-count row: the other rows exist in fixed point only (33 MB instead of
+    // 40 GB at config 4)
+    bool compact() const { return rows == Rows::FastPlanes || rows == Rows::Q; }
+};
+
+TablePlan plan_table(const scde_b200_ctx *ctx, const TableRequest &r) {
+    TablePlan pl;
+    const bool fits = r.K <= KP_TILED;  // the table's ld is KP_TILED
+    pl.zero_base = r.zero_base && fits && (r.probe || ctx->opt.zero_base);
+    pl.fast = r.models->fast_theta && !r.models->local_theta && fits;
+    pl.planes = r.fixed_point && pl.zero_base && r.K <= Q_MAX_K;
+    pl.bounds = pl.planes && (r.bounds || (ctx->opt.prune_pieces && r.models->C >= PRUNE_MIN_CELLS));
+    pl.modes = r.modes;
+    pl.rows = pl.fast ? Rows::Fast : Rows::General;
+    if (pl.planes && pl.fast && ctx->opt.fused_fixed_point)
+        pl.rows = !pl.modes && ctx->opt.lp_rows_kernel == 0 ? Rows::Q : Rows::FastPlanes;
+    return pl;
+}
+
 inline int table_ld(int K) { return K <= KP_TILED ? KP_TILED : round_up(K, 8); }
 
 struct LpTable {
     int n_cells = 0, n_genes = 0, K = 0, ld = 0, ld_ridx = 0;
     int64_t n_rows = 0;
     double sentinel = 0;
+    TablePlan plan;  // of the table built last (begin_table)
+    CellPrep prep{};
     DBuf<int32_t> row_off, row_x, row_mode, row_cell, row_snap, ridx, n_unique, err, zero_row, based;
     DBuf<double> table, mu, lcfp, lcfpr, theta, maxcfp, cfp, l1, l2, rowc, scfp;
     DBuf<int8_t> q;      // fixed-point planes of the table (contract_i8.cu), [n_rows][q_row_bytes(K)]
@@ -171,18 +228,6 @@ struct LpTable {
     DBuf<int8_t> qb;        // [n_rows][Q_BW] bound rows of the fixed-point table (pruned contraction)
     DBuf<uint32_t> dedup_bits;  // per-cell bitmaps between the two dedup passes
     DBuf<unsigned long long> work_counter;  // chunk counter of the fixed-point row kernel
-    bool want_q = false, has_q = false;
-    bool want_bounds = false;  // bound rows whatever the size (scde_b200_probe_table_bounds)
-    bool has_bounds = false;   // t.qb holds the bound rows of the fixed-point table
-    bool f64_rows = true;  // false: the FP64 rows of non-zero counts were not stored (planes only)
-    bool want_modes = true;  // row_mode (argmax of every row) is needed: only for return.individual.posterior.modes
-    bool fast_theta = false;  // every corr.theta finite and > 0, no local-theta fit: constant-theta fast path
-    // zero-base form: rows of non-zero counts hold lp(x) - lp(0) of their cell, the zero-count rows lp(0) itself, and
-    // the contraction only visits the cells whose count is non-zero (boot_contract.cu)
-    bool zero_base = false;
-    // the FP64 table holds one row per CELL (its zero-count row, at the cell's index) instead of one per table row: set by
-    // reserve_rows when the fixed-point planes come from the row kernel itself, which stores no other FP64 row
-    bool zero_compact = false;
 };
 
 #define TRY(x)                          \
@@ -200,43 +245,22 @@ struct LpTable {
         SCDE_CUDA(cudaSetDevice((ctx)->device));                        \
     } while (0)
 
-// What fill_table decides once per table and the row-level launches need: which kernels, which outputs.
-// Pruning (DESIGN.md 4.3) pays where a joint has at least this many cells: measured on one B200 (1000 W), config 3 (1000
-// cells per joint) was 3.0 ms per step slower with it (bound pass and bound rows cost more than the 27 % of the gather they
-// removed), config 4 (5000) 7.7 ms faster.  The bound rows are only written for tables of at least as many cells.
-constexpr int PRUNE_MIN_CELLS = 2500;
-
-struct TablePlan {
-    bool fast = false;     // constant-theta fast row kernel
-    bool q_any = false;    // the table also exists in fixed point (tcgen05 contraction)
-    bool q_fused = false;  // ... emitted by the row kernel itself; the FP64 rows of non-zero counts are then not stored
-    CellPrep prep{};
-    void *rowc = nullptr;
-    int32_t *rmode = nullptr;
-    int8_t *qf = nullptr;
-    uint32_t *qr = nullptr;
-    int8_t *qb = nullptr;
-    bool bounds = false;   // the table also gets its bound rows
-};
-
-TablePlan plan_table(const scde_b200_ctx *ctx, const LpTable &t, int local_theta) {
-    TablePlan pl;
-    pl.fast = t.fast_theta && !local_theta && t.K <= KP_TILED;
-    pl.q_any = t.want_q && t.zero_base && t.ld == KP_TILED && t.K <= Q_MAX_K;
-    pl.q_fused = pl.q_any && pl.fast && ctx->opt.fused_fixed_point;
-    pl.bounds = pl.q_any && (t.want_bounds || (ctx->opt.prune_pieces && t.n_cells >= PRUNE_MIN_CELLS));
-    return pl;
-}
-
-// per-cell buffers (independent of the number of table rows) + the per-cell grid vectors
-int prepare_cells(scde_b200_ctx *ctx, LpTable &t, TablePlan &pl, const double *models_dev, int ld_models,
-                  const double *mag_dev, int local_theta, int sqlogit) {
+// A table is built in steps, which the chunked front of the one-shot call interleaves with its count chunks: begin_table
+// (the plan, the shape and the per-cell grid vectors), reserve_rows (the row buffers for a capacity, once it is known),
+// table_rows for ranges of cells (t.row_off / t.row_x of their rows in place) and finish_table (the quantize pass).
+int begin_table(scde_b200_ctx *ctx, LpTable &t, const TableRequest &r, StageTimer *tm) {
     cudaStream_t st = ctx->stream;
+    const TablePlan &pl = t.plan = plan_table(ctx, r);
+    const ModelSet &ms = *r.models;
+    t.n_cells = ms.C;
+    t.K = r.K;
+    t.ld = table_ld(r.K);
+    t.sentinel = -DBL_MAX / r.clamp_n / 1.1;
     const size_t cl = (size_t)t.n_cells * t.ld;
     SCDE_CUDA(t.mu.ensure(cl));
     SCDE_CUDA(t.lcfp.ensure(cl));
     SCDE_CUDA(t.lcfpr.ensure(cl));
-    if (local_theta) SCDE_CUDA(t.theta.ensure(cl));
+    if (ms.local_theta) SCDE_CUDA(t.theta.ensure(cl));
     SCDE_CUDA(t.maxcfp.ensure(t.n_cells));
     if (pl.fast) {
         SCDE_CUDA(t.cfp.ensure(cl));
@@ -244,96 +268,83 @@ int prepare_cells(scde_b200_ctx *ctx, LpTable &t, TablePlan &pl, const double *m
         SCDE_CUDA(t.l2.ensure(cl));
         SCDE_CUDA(t.scfp.ensure((size_t)t.n_cells));
     }
-    if (t.zero_base) {
+    if (pl.zero_base) {
         SCDE_CUDA(t.zero_row.ensure((size_t)t.n_cells));
         SCDE_CUDA(t.based.ensure((size_t)t.n_cells));
     }
-    pl.prep = CellPrep{t.mu.p, t.lcfp.p, t.lcfpr.p, local_theta ? t.theta.p : nullptr, t.maxcfp.p, t.ld,
-                       pl.fast ? t.cfp.p : nullptr, pl.fast ? t.l1.p : nullptr, pl.fast ? t.l2.p : nullptr,
-                       pl.fast ? t.scfp.p : nullptr};
-    SCDE_CUDA(launch_cell_prep(models_dev, ld_models, t.n_cells, mag_dev, t.K, local_theta, sqlogit, pl.prep, st));
+    t.prep = CellPrep{t.mu.p, t.lcfp.p, t.lcfpr.p, ms.local_theta ? t.theta.p : nullptr, t.maxcfp.p, t.ld,
+                      pl.fast ? t.cfp.p : nullptr, pl.fast ? t.l1.p : nullptr, pl.fast ? t.l2.p : nullptr,
+                      pl.fast ? t.scfp.p : nullptr};
+    const int e0 = tm ? tm->begin(st) : -1;
+    SCDE_CUDA(launch_cell_prep(ms.m.p, ms.C, t.n_cells, r.mag, t.K, ms.local_theta, ms.sqlogit, t.prep, st));
+    if (tm) tm->end(SCDE_B200_T_LPTABLE, e0, st, 1);
     return SCDE_B200_OK;
 }
 
-// per-row buffers for `rows` table rows
-int reserve_rows(LpTable &t, TablePlan &pl, size_t rows) {
-    t.zero_compact = pl.q_fused && t.zero_base;  // 33 MB instead of 40 GB at config 4
-    SCDE_CUDA(t.table.ensure((t.zero_compact ? (size_t)t.n_cells : rows) * t.ld));
+int reserve_rows(LpTable &t, size_t rows) {
+    const TablePlan &pl = t.plan;
+    SCDE_CUDA(t.table.ensure((pl.compact() ? (size_t)t.n_cells : rows) * t.ld));
     SCDE_CUDA(t.row_mode.ensure(rows));
     SCDE_CUDA(t.row_cell.ensure(rows));
     if (pl.fast) {
         SCDE_CUDA(t.rowc.ensure(4 * rows));
         SCDE_CUDA(t.row_snap.ensure(rows));
     }
-    if (pl.q_any) {
+    if (pl.planes) {
         SCDE_CUDA(t.q.ensure(rows * q_row_bytes(t.K)));
         SCDE_CUDA(t.qrange.ensure(rows));
         if (pl.bounds) SCDE_CUDA(t.qb.ensure(rows * Q_BW));
         SCDE_CUDA(t.work_counter.ensure(1));
     }
-    pl.rowc = pl.fast ? (void *)t.rowc.p : nullptr;
-    pl.rmode = t.want_modes ? t.row_mode.p : nullptr;
-    pl.qf = pl.q_fused ? t.q.p : nullptr;
-    pl.qr = pl.q_fused ? t.qrange.p : nullptr;
-    pl.qb = pl.q_fused && pl.bounds ? t.qb.p : nullptr;
-    t.has_bounds = pl.bounds;
     return SCDE_B200_OK;
 }
 
-// the row-level kernels for the cells of `cr` (their rows are read from t.row_off on the device); returns the number of
-// launches through *nl
-int launch_table_rows(scde_b200_ctx *ctx, const LpTable &t, const TablePlan &pl, CellRange cr, const double *models_dev,
-                      int ld_models, int local_theta, int *nl) {
+// the rows of the cells of cr (their rows are read from t.row_off on the device), from the models the table was begun with
+int table_rows(scde_b200_ctx *ctx, LpTable &t, const ModelSet &ms, CellRange cr, StageTimer *tm) {
     cudaStream_t st = ctx->stream;
+    const TablePlan &pl = t.plan;
     const int n = cr.c1 - cr.c0;
+    const RowArgs a{ms.m.p, ms.C, t.row_off.p, t.row_cell.p, t.row_x.p, t.prep, t.K, t.sentinel, t.table.p, t.ld,
+                    pl.fast, pl.fast ? (void *)t.rowc.p : nullptr, t.row_snap.p, ms.local_theta, t.zero_row.p, t.based.p,
+                    pl.compact()};
+    int32_t *rmode = pl.modes ? t.row_mode.p : nullptr;
+    const RowPlanes q{t.q.p, t.qrange.p, pl.bounds ? t.qb.p : nullptr};
+    const int e0 = tm ? tm->begin(st) : -1;
     SCDE_CUDA(launch_row_cell(t.row_off.p, cr, t.row_cell.p, st));
-    ++*nl;
-    if (pl.fast) {
-        SCDE_CUDA(launch_row_consts(models_dev, ld_models, t.row_off.p, cr, t.row_cell.p, t.row_x.p, pl.rowc, t.row_snap.p,
-                                    pl.prep, t.K, st));
-        ++*nl;
-    }
-    if (t.zero_base) {
+    if (pl.fast)
+        SCDE_CUDA(launch_row_consts(ms.m.p, ms.C, t.row_off.p, cr, t.row_cell.p, t.row_x.p, t.rowc.p, t.row_snap.p, t.prep,
+                                    t.K, st));
+    if (pl.zero_base) {
         SCDE_CUDA(launch_zero_rows(t.row_off.p + cr.c0, t.row_x.p, n, t.zero_row.p + cr.c0, cr.row_cap, st));
-        SCDE_CUDA(launch_lp_rows(models_dev, ld_models, cr, t.row_off.p, t.row_cell.p, t.row_x.p, pl.prep, t.K, local_theta,
-                                 t.sentinel, t.table.p, t.ld, pl.rmode, 1, t.zero_row.p, nullptr, pl.rowc, t.row_snap.p, 1, pl.qf, pl.qr,
-                                 st, 0, nullptr, t.zero_compact, pl.qb));
+        SCDE_CUDA(launch_zero_count_rows(a, cr, rmode, pl.compact() ? q : RowPlanes{}, st));
         SCDE_CUDA(launch_based_flags(t.table.p, t.ld, t.K, t.sentinel, t.zero_row.p + cr.c0, n, t.based.p + cr.c0, st,
-                                     t.zero_compact ? cr.c0 : -1));
-        SCDE_CUDA(launch_lp_rows(models_dev, ld_models, cr, t.row_off.p, t.row_cell.p, t.row_x.p, pl.prep, t.K, local_theta,
-                                 t.sentinel, t.table.p, t.ld, pl.rmode, 2, t.zero_row.p, t.based.p, pl.rowc, t.row_snap.p,
-                                 pl.q_fused ? 0 : 1, pl.qf, pl.qr, st, ctx->opt.lp_rows_kernel == 1, t.work_counter.p,
-                                 t.zero_compact, pl.qb));
-        *nl += 4;
+                                     pl.compact() ? cr.c0 : -1));
+        if (pl.rows == Rows::Q)
+            SCDE_CUDA(launch_q_rows(a, cr, q, t.work_counter.p, st));
+        else
+            SCDE_CUDA(launch_nonzero_rows(a, cr, rmode, pl.rows == Rows::FastPlanes ? q : RowPlanes{}, st));
     } else {
-        SCDE_CUDA(launch_lp_rows(models_dev, ld_models, cr, t.row_off.p, t.row_cell.p, t.row_x.p, pl.prep, t.K, local_theta,
-                                 t.sentinel, t.table.p, t.ld, pl.rmode, 0, nullptr, nullptr, pl.rowc, t.row_snap.p, 1, nullptr, nullptr,
-                                 st));
-        ++*nl;
+        SCDE_CUDA(launch_dense_rows(a, cr, rmode, st));
     }
+    if (tm) tm->end(SCDE_B200_T_LPTABLE, e0, st, 1 + pl.fast + (pl.zero_base ? 4 : 1));
     return SCDE_B200_OK;
 }
 
-// rows of the table from the per-cell model rows; t.row_off / t.row_x / t.n_rows must be set
-int fill_table(scde_b200_ctx *ctx, LpTable &t, const double *models_dev, int ld_models, const double *mag_dev,
-               int local_theta, int sqlogit, StageTimer *tm) {
+int finish_table(scde_b200_ctx *ctx, LpTable &t, StageTimer *tm) {
     cudaStream_t st = ctx->stream;
-    TablePlan pl = plan_table(ctx, t, local_theta);
-    TRY(reserve_rows(t, pl, (size_t)t.n_rows));
-    int e0 = tm ? tm->begin(st) : -1;
-    int nl = 1;
-    TRY(prepare_cells(ctx, t, pl, models_dev, ld_models, mag_dev, local_theta, sqlogit));
-    // fixed-point planes for the tcgen05 contraction: emitted by the fast row kernel itself (the FP64 rows of non-zero
-    // counts are then not stored at all), by a separate pass over the FP64 table for the general kernel
-    TRY(launch_table_rows(ctx, t, pl, CellRange{0, t.n_cells, (int64_t)t.n_rows}, models_dev, ld_models, local_theta, &nl));
-    t.has_q = pl.q_any;
-    t.f64_rows = !(pl.q_fused && t.zero_base);
-    if (pl.q_any && !pl.q_fused) {
-        SCDE_CUDA(launch_quantize_rows(t.table.p, t.ld, t.K, t.n_rows, t.q.p, t.qrange.p, pl.bounds ? t.qb.p : nullptr, st));
-        ++nl;
-    }
-    if (tm) tm->end(SCDE_B200_T_LPTABLE, e0, st, nl);
+    if (!t.plan.planes || t.plan.compact()) return SCDE_B200_OK;  // planes from a pass over the FP64 table
+    const int e0 = tm ? tm->begin(st) : -1;
+    SCDE_CUDA(launch_quantize_rows(t.table.p, t.ld, t.K, t.n_rows, t.q.p, t.qrange.p, t.plan.bounds ? t.qb.p : nullptr, st));
+    if (tm) tm->end(SCDE_B200_T_LPTABLE, e0, st, 1);
     return SCDE_B200_OK;
+}
+
+// the table r asks for, over t.n_rows rows
+int fill_table(scde_b200_ctx *ctx, LpTable &t, const TableRequest &r, StageTimer *tm) {
+    TRY(begin_table(ctx, t, r, tm));
+    TRY(reserve_rows(t, (size_t)t.n_rows));
+    TRY(table_rows(ctx, t, *r.models, CellRange{0, t.n_cells, t.n_rows}, tm));
+    return finish_table(ctx, t, tm);
 }
 
 // The contraction kernel of one call, resolved from the context's options once and passed down.  I8: tcgen05 on the
@@ -354,6 +365,32 @@ ContractChoice contraction_choice(const scde_b200_ctx *ctx) {
     }
 }
 
+// the index buffers of G genes x C cells, and the dedup error word zeroed on the stream
+int index_buffers(scde_b200_ctx *ctx, LpTable &t, int G, int C) {
+    t.n_genes = G;
+    t.ld_ridx = C;
+    SCDE_CUDA(t.n_unique.ensure(C));
+    SCDE_CUDA(t.row_off.ensure((size_t)C + 1));
+    SCDE_CUDA(t.err.ensure(1));
+    SCDE_CUDA(t.ridx.ensure((size_t)G * C));
+    SCDE_CUDA(t.dedup_bits.ensure(dedup_scratch_words(C)));
+    SCDE_CUDA(cudaMemsetAsync(t.err.p, 0, sizeof(int32_t), ctx->stream));
+    return SCDE_B200_OK;
+}
+
+// the dedup passes' error word, read back
+int dedup_error(int32_t err) {
+    if (err & 1) {
+        set_error("negative count in the count matrix");
+        return SCDE_B200_EINVAL;
+    }
+    if (err & 2) {
+        set_error("a cell has >= 32768 distinct count values among the processed genes (hash capacity)");
+        return SCDE_B200_ELIMIT;
+    }
+    return SCDE_B200_OK;
+}
+
 // unique-count indices from raw counts (device, column-major, leading dimension ldc, genes [g0, g0+G)).
 // known_cap > 0: the row buffers already hold known_cap rows (an earlier run of the same job) -- nothing is read back, the
 // emit pass and the row kernels take their bounds from row_off on the device and stop at the capacity; the caller
@@ -361,16 +398,8 @@ ContractChoice contraction_choice(const scde_b200_ctx *ctx) {
 int index_from_counts(scde_b200_ctx *ctx, LpTable &t, const int32_t *counts_dev, int64_t ldc, int g0, int G, int C,
                       StageTimer *tm, int64_t known_cap = 0) {
     cudaStream_t st = ctx->stream;
-    t.n_cells = C;
-    t.n_genes = G;
-    t.ld_ridx = C;
-    SCDE_CUDA(t.n_unique.ensure(C));
-    SCDE_CUDA(t.row_off.ensure((size_t)C + 1));
-    SCDE_CUDA(t.err.ensure(1));
-    SCDE_CUDA(t.ridx.ensure((size_t)G * C));
     int e0 = tm ? tm->begin(st) : -1;
-    SCDE_CUDA(cudaMemsetAsync(t.err.p, 0, sizeof(int32_t), st));
-    SCDE_CUDA(t.dedup_bits.ensure(dedup_scratch_words(C)));
+    TRY(index_buffers(ctx, t, G, C));
     SCDE_CUDA(launch_dedup_count(counts_dev, ldc, g0, G, C, t.n_unique.p, t.err.p, t.dedup_bits.p, st));
     SCDE_CUDA(launch_exclusive_scan(t.n_unique.p, t.row_off.p, C, nullptr, st));
     int64_t cap = known_cap;
@@ -379,14 +408,7 @@ int index_from_counts(scde_b200_ctx *ctx, LpTable &t, const int32_t *counts_dev,
         SCDE_CUDA(cudaMemcpyAsync(&total, t.row_off.p + C, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
         SCDE_CUDA(cudaMemcpyAsync(&err, t.err.p, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
         SCDE_CUDA(cudaStreamSynchronize(st));  // the table is sized by the number of distinct (cell, count) pairs
-        if (err & 1) {
-            set_error("negative count in the count matrix");
-            return SCDE_B200_EINVAL;
-        }
-        if (err & 2) {
-            set_error("a cell has >= 32768 distinct count values among the processed genes (hash capacity)");
-            return SCDE_B200_ELIMIT;
-        }
+        TRY(dedup_error(err));
         cap = total;
     }
     t.n_rows = cap;
@@ -555,7 +577,7 @@ int contract_joint_fp64(scde_b200_ctx *ctx, Contraction kernel, const LpTable &t
                         JointScratch &scr, const double *Z, int n_w_rows, int n_boot, const DrawSets &sets, double scale,
                         double *jp_dev, int ld_jp, StageTimer *tm) {
     cudaStream_t st = ctx->stream;
-    if (!t.f64_rows) {
+    if (t.plan.compact()) {
         set_error("internal: the table was built in fixed point only but the FP64 contraction kernel was selected");
         return SCDE_B200_EINVAL;
     }
@@ -605,9 +627,9 @@ int run_joint(scde_b200_ctx *ctx, ContractChoice k, const LpTable &t, const int3
     const int n_w_rows = round_up(n_list + 1, 16);  // at least one all-zero row after the cells (list padding)
     const int passes = (n_boot + WP_TILED - 1) / WP_TILED;
     const int ld_lst = round_up(n_list, 32);
-    const bool zb = t.zero_base && t.ld <= KP_TILED;
+    const bool zb = t.plan.zero_base;
     auto i8_for = [&](const Joint &jt) {
-        return zb && t.has_q && k.kernel == Contraction::I8 && contract_i8_supported(t.K, t.ld, ld_lst, jt.D);
+        return t.plan.planes && k.kernel == Contraction::I8 && contract_i8_supported(t.K, t.ld, ld_lst, jt.D);
     };
     if (n_joints > 1 && !(i8_for(joints[0]) && i8_for(joints[1]) && ctx->opt.twin_batch_joints)) {
         for (int j = 0; j < n_joints; ++j)
@@ -651,7 +673,7 @@ int run_joint(scde_b200_ctx *ctx, ContractChoice k, const LpTable &t, const int3
             for (int s = 0; s < S; ++s)
                 SCDE_CUDA(launch_base_sum(t.table.p, t.ld, t.zero_row.p, t.based.p, cell_ids_dev, n_list,
                                           scr.W[j].p + s * w_set, n_w_rows, n_boot, scr.Z[j].p + s * z_set, scr.zpart.p, st,
-                                          t.zero_compact));
+                                          t.plan.compact()));
         // W8 of all sets in one conversion: the sets' blocks are consecutive rows
         if (i8) SCDE_CUDA(launch_w_to_i8(scr.W[j].p, S * n_w_rows, n_boot, scr.W8[j].p, status, st));
     }
@@ -661,7 +683,7 @@ int run_joint(scde_b200_ctx *ctx, ContractChoice k, const LpTable &t, const int3
         return contract_joint_fp64(ctx, k.kernel, t, lists, scr, zb ? scr.Z[0].p : nullptr, n_w_rows, n_boot, sets, scale,
                                    joints[0].jp_dev, ld_jp, tm);
     return contract_joint_i8(ctx, t, lists, scr, n_w_rows, n_boot, sets, scale, joints, n_joints, ld_jp, hot_rank, status, tm,
-                             t.has_bounds && ctx->opt.prune_pieces && n_list >= PRUNE_MIN_CELLS,
+                             t.plan.bounds && ctx->opt.prune_pieces && n_list >= PRUNE_MIN_CELLS,
                              count_entries ? scr.total.p + 1 : nullptr);
 }
 
@@ -767,13 +789,6 @@ std::vector<int32_t> zero_slice(const int32_t *zero_index, int n_zero, int g0, i
     return zi;
 }
 
-// One set of per-cell error models on the device (C x 12, column-major) and what building table rows from it needs
-struct ModelSet {
-    DBuf<double> m;
-    int C = 0, local_theta = 0, sqlogit = 0;
-    bool fast_theta = false;  // every corr.theta finite and > 0, no local-theta fit
-};
-
 int upload_models(ModelSet &s, const double *models, int C, int local_theta, int sqlogit, cudaStream_t st) {
     s.C = C;
     s.local_theta = local_theta;
@@ -782,21 +797,12 @@ int upload_models(ModelSet &s, const double *models, int C, int local_theta, int
     return upload(s.m, models, (size_t)C * 12, st);
 }
 
-// the table rows from the model set ms (index and row ids must be in place)
-int fill_rows(scde_b200_ctx *ctx, LpTable &t, const ModelSet &ms, const double *mag_dev, StageTimer *tm) {
-    t.fast_theta = ms.fast_theta;
-    return fill_table(ctx, t, ms.m.p, ms.C, mag_dev, ms.local_theta, ms.sqlogit, tm);
-}
-
-// the table of a differential-expression call over C cells and a K-point grid
-void init_table(const scde_b200_ctx *ctx, ContractChoice k, LpTable &t, int K, int C, bool fast_theta) {
-    t.K = K;
-    t.ld = table_ld(K);
-    t.sentinel = -DBL_MAX / C / 1.1;
-    t.fast_theta = fast_theta;
-    t.zero_base = t.ld <= KP_TILED && ctx->opt.zero_base;
-    t.want_q = k.kernel == Contraction::I8;
-    t.want_modes = false;
+// the table of a differential-expression call: the cells of the model set ms on a K-point grid, for the contraction k
+TableRequest diff_table(const ModelSet &ms, const double *mag_dev, int K, ContractChoice k) {
+    TableRequest r{&ms, mag_dev, K, ms.C};
+    r.zero_base = true;
+    r.fixed_point = k.kernel == Contraction::I8;
+    return r;
 }
 
 int workspace_busy(const scde_b200_ctx *ctx) {
@@ -1243,19 +1249,17 @@ int scde_b200_cell_table(scde_b200_ctx *ctx, const double *model_row12, const in
     }
     cudaStream_t st = ctx->stream;
     LpTable t;
-    t.n_cells = 1;
-    t.K = n_grid;
-    t.ld = table_ld(n_grid);
     t.n_rows = n_counts;
-    t.sentinel = -DBL_MAX / n_cells_for_clamp / 1.1;
-    t.fast_theta = !local_theta && theta_all_regular(model_row12, 1, 1);
-    DBuf<double> d_models, d_mag;
-    TRY(upload(d_models, model_row12, 12, st));
+    ModelSet ms;
+    DBuf<double> d_mag;
+    TRY(upload_models(ms, model_row12, 1, local_theta, square_logit_conc, st));
     TRY(upload(d_mag, magnitudes, (size_t)n_grid, st));
     int32_t off[2] = {0, n_counts};
     TRY(upload(t.row_off, off, 2, st));
     TRY(upload(t.row_x, unique_counts, (size_t)n_counts, st));
-    TRY(fill_table(ctx, t, d_models.p, 1, d_mag.p, local_theta, square_logit_conc, nullptr));
+    TableRequest r{&ms, d_mag.p, n_grid, n_cells_for_clamp};
+    r.modes = true;
+    TRY(fill_table(ctx, t, r, nullptr));
     if (n_counts > 0) {
         SCDE_CUDA(cudaMemcpy2DAsync(out, sizeof(double) * n_grid, t.table.p, sizeof(double) * t.ld, sizeof(double) * n_grid,
                                     n_counts, cudaMemcpyDeviceToHost, st));
@@ -1308,28 +1312,23 @@ int scde_b200_probe_table_bounds(scde_b200_ctx *ctx, const double *models, int32
     }
     cudaStream_t st = ctx->stream;
     LpTable t;
-    t.n_cells = n_cells;
-    t.K = n_grid;
-    t.ld = table_ld(n_grid);
     t.n_rows = ucl_offsets[n_cells];
-    t.sentinel = -DBL_MAX / n_cells_for_clamp / 1.1;
-    t.fast_theta = !local_theta && theta_all_regular(models, n_cells, n_cells);
-    t.zero_base = true;
-    t.want_q = true;
-    t.want_bounds = qbound_out != nullptr;
-    t.want_modes = false;
-    DBuf<double> d_models, d_mag;
-    TRY(upload(d_models, models, (size_t)n_cells * 12, st));
+    ModelSet ms;
+    DBuf<double> d_mag;
+    TRY(upload_models(ms, models, n_cells, local_theta, square_logit_conc, st));
     TRY(upload(d_mag, magnitudes, (size_t)n_grid, st));
     TRY(upload(t.row_off, ucl_offsets, (size_t)n_cells + 1, st));
     TRY(upload(t.row_x, ucl_flat, (size_t)t.n_rows, st));
-    TRY(fill_table(ctx, t, d_models.p, n_cells, d_mag.p, local_theta, square_logit_conc, nullptr));
-    if (!t.has_q) {
+    TableRequest r{&ms, d_mag.p, n_grid, n_cells_for_clamp};
+    r.zero_base = r.fixed_point = r.probe = true;
+    r.bounds = qbound_out != nullptr;
+    TRY(fill_table(ctx, t, r, nullptr));
+    if (!t.plan.planes) {
         set_error("probe_table: the table was built without fixed-point planes");
         return SCDE_B200_EINVAL;
     }
     SCDE_CUDA(cudaMemcpyAsync(q_out, t.q.p, (size_t)t.n_rows * q_row_bytes(n_grid), cudaMemcpyDeviceToHost, st));
-    if (qbound_out && t.has_bounds) SCDE_CUDA(cudaMemcpyAsync(qbound_out, t.qb.p, (size_t)t.n_rows * Q_BW, cudaMemcpyDeviceToHost, st));
+    if (qbound_out && t.plan.bounds) SCDE_CUDA(cudaMemcpyAsync(qbound_out, t.qb.p, (size_t)t.n_rows * Q_BW, cudaMemcpyDeviceToHost, st));
     SCDE_CUDA(cudaMemcpyAsync(row_range_out, t.qrange.p, sizeof(uint32_t) * t.n_rows, cudaMemcpyDeviceToHost, st));
     SCDE_CUDA(cudaMemcpyAsync(zero_row_out, t.zero_row.p, sizeof(int32_t) * n_cells, cudaMemcpyDeviceToHost, st));
     SCDE_CUDA(cudaMemcpyAsync(based_out, t.based.p, sizeof(int32_t) * n_cells, cudaMemcpyDeviceToHost, st));
@@ -1342,7 +1341,7 @@ int scde_b200_probe_table_bounds(scde_b200_ctx *ctx, const double *models, int32
             for (int k = 0; k < n_grid; ++k) dst[k] = std::nan("");
             continue;
         }
-        const size_t slot = t.zero_compact ? (size_t)c : (size_t)zr;
+        const size_t slot = t.plan.compact() ? (size_t)c : (size_t)zr;
         SCDE_CUDA(cudaMemcpyAsync(dst, t.table.p + slot * t.ld, sizeof(double) * n_grid, cudaMemcpyDeviceToHost, st));
     }
     SCDE_CUDA(cudaStreamSynchronize(st));
@@ -1385,30 +1384,27 @@ static int log_boot_impl(scde_b200_ctx *ctx, const double *models, int32_t n_cel
     }
     if (n_genes == 0) return SCDE_B200_OK;
     LpTable t;
-    t.n_cells = n_cells;
     t.n_genes = n_genes;
-    t.K = n_grid;
-    t.ld = table_ld(n_grid);
     t.ld_ridx = n_cells;
     t.n_rows = ucl_offsets[n_cells];
     const double minlogprob = -DBL_MAX / n_cells / 1.1;  // src/jpmatLogBoot.cpp:127,372
-    t.sentinel = -DBL_MAX / (double)(D > n_cells ? D : n_cells) / 1.1;
-    t.fast_theta = !local_theta && theta_all_regular(models, n_cells, n_cells);
-    t.zero_base = !post_flag && !ensemble && t.ld <= KP_TILED && ctx->opt.zero_base;
-    t.want_q = k.kernel == Contraction::I8 && n_boot > 0;
-    t.want_modes = modes_flag != 0;
-    DBuf<double> d_models, d_mag, d_jp, d_out, d_rs;
+    ModelSet ms;
+    DBuf<double> d_mag, d_jp, d_out, d_rs;
     DBuf<int32_t> d_uci, d_boot, status;
     SCDE_CUDA(status.ensure(1));
     SCDE_CUDA(cudaMemsetAsync(status.p, 0, sizeof(int32_t), st));
-    TRY(upload(d_models, models, (size_t)n_cells * 12, st));
+    TRY(upload_models(ms, models, n_cells, local_theta, square_logit_conc, st));
     TRY(upload(d_mag, magnitudes, (size_t)n_grid, st));
     TRY(upload(t.row_off, ucl_offsets, (size_t)n_cells + 1, st));
     TRY(upload(t.row_x, ucl_flat, (size_t)t.n_rows, st));
     TRY(upload(d_uci, uci, (size_t)n_genes * n_cells, st));
     SCDE_CUDA(t.ridx.ensure((size_t)n_genes * n_cells));
     SCDE_CUDA(launch_uci_to_ridx(d_uci.p, n_genes, n_cells, t.row_off.p, t.ridx.p, t.ld_ridx, st));
-    TRY(fill_table(ctx, t, d_models.p, n_cells, d_mag.p, local_theta, square_logit_conc, nullptr));
+    TableRequest r{&ms, d_mag.p, n_grid, D > n_cells ? D : n_cells};
+    r.zero_base = !post_flag && !ensemble;
+    r.fixed_point = k.kernel == Contraction::I8 && n_boot > 0;
+    r.modes = modes_flag != 0;
+    TRY(fill_table(ctx, t, r, nullptr));
     const int ld_jp = t.ld;
     SCDE_CUDA(d_jp.ensure((size_t)n_genes * ld_jp));
     JointScratch scr;
@@ -2011,7 +2007,6 @@ struct scde_b200_diff_job {
     int split_chunks = 0;            // > 0: the chunks [0, split_chunks) hold every cell of the first group, whose joint
                                      // runs before the rest of the front (so it hides the second half of the upload)
     int64_t front_cap = 0;           // row capacity chosen by the chunked front
-    TablePlan front_plan;            // the front's table plan (buffers bound in its first phase)
     const int32_t *boot_ptr[4] = {nullptr, nullptr, nullptr, nullptr};  // draws as the device reads them
     std::vector<int32_t> ids[2];                 // cells of the two groups
     std::unique_ptr<int32_t[]> gen[4];           // generated draws (resident job), alive until their uploads have completed
@@ -2196,7 +2191,7 @@ static int gene_range(const scde_b200_diff_args *a, int *g0, int *g1) {
 }
 
 // defer_counts: the count matrix is not copied here (the one-shot call overlaps its upload with the table build)
-static int diff_upload_impl(scde_b200_ctx *ctx, ContractChoice k, const scde_b200_diff_args *a, int32_t want_posteriors,
+static int diff_upload_impl(scde_b200_ctx *ctx, const scde_b200_diff_args *a, int32_t want_posteriors,
                             scde_b200_diff_job **out, bool defer_counts) {
     if (!a || !out) return SCDE_B200_EINVAL;
     *out = nullptr;
@@ -2315,7 +2310,6 @@ static int diff_upload_impl(scde_b200_ctx *ctx, ContractChoice k, const scde_b20
         JCUDA(j->az.ensure((size_t)G));
         if (want_posteriors) JCUDA(j->ws->apost.ensure((size_t)G * lda));
     }
-    init_table(ctx, k, j->ws->table, K, C, j->models.fast_theta);  // the chunked front's table plan reads models' fast_theta
     JCUDA(cudaStreamSynchronize(st));
     // last: the small uploads above share the one H2D copy engine with these 1.2 GB and would queue behind them
     if (defer_counts) JTRY(start_count_copies(ctx, j, a->counts + g0, a->n_genes));
@@ -2333,19 +2327,17 @@ static int diff_upload_impl(scde_b200_ctx *ctx, ContractChoice k, const scde_b20
 // at the capacity and *done stays false: the caller rebuilds index and table the classic way from the resident counts.
 // phase 0: the chunks [0, split_chunks) -- all of them without a split; phase 1: the rest (split front only).  A phase
 // returns with the compute stream idle and its rows checked against the capacity, so the caller may queue a joint on them.
-static int front_chunked(scde_b200_ctx *ctx, scde_b200_diff_job *j, int phase, bool *done) {
+static int front_chunked(scde_b200_ctx *ctx, scde_b200_diff_job *j, ContractChoice k, int phase, bool *done) {
     *done = false;
     LpTable &t = j->ws->table;
     const int G = j->G, C = j->C;
     cudaStream_t st = ctx->stream;
     StageTimer &tm = j->timer;
-    t.n_cells = C;
-    t.n_genes = G;
-    t.ld_ridx = C;
-    if (phase == 0) j->front_plan = plan_table(ctx, t, j->models.local_theta);
-    TablePlan &pl = j->front_plan;  // prepare_cells and reserve_rows bind its buffers in phase 0
-    // the copies are already in flight (start_count_copies); every path below waits for them on the compute stream
-    const bool pipelined = pl.q_fused && t.zero_base && C >= 64 * j->copy_chunks && ctx->opt.pipeline_front;
+    const TableRequest req = diff_table(j->models, j->mag.p, j->K, k);
+    // the copies are already in flight (start_count_copies); every path below waits for them on the compute stream.  Only
+    // the compact table is built chunk by chunk: its rows need no pass after the last chunk, and a row capacity estimated
+    // too large costs fixed-point rows only.
+    const bool pipelined = plan_table(ctx, req).compact() && C >= 64 * j->copy_chunks && ctx->opt.pipeline_front;
     if (!pipelined) {
         j->split_chunks = 0;
         for (int i = 0; i < j->copy_chunks; ++i) SCDE_CUDA(cudaStreamWaitEvent(st, ctx->copy_events[i], 0));
@@ -2374,15 +2366,8 @@ static int front_chunked(scde_b200_ctx *ctx, scde_b200_diff_job *j, int phase, b
     double tr_first = 0, tr_queued = 0, tr_draws = 0, tr_front = 0, tr_copy = 0;
     int e0 = 0;
     if (phase == 0) {
-        FCUDA(t.n_unique.ensure(C));
-        FCUDA(t.row_off.ensure((size_t)C + 1));
-        FCUDA(t.err.ensure(1));
-        FCUDA(t.ridx.ensure((size_t)G * C));
-        FCUDA(t.dedup_bits.ensure(dedup_scratch_words(C)));
-        FCUDA(cudaMemsetAsync(t.err.p, 0, sizeof(int32_t), st));
-        e0 = tm.begin(st);
-        FTRY(prepare_cells(ctx, t, pl, j->models.m.p, C, j->mag.p, j->models.local_theta, j->models.sqlogit));
-        tm.end(SCDE_B200_T_LPTABLE, e0, st, 1);
+        FTRY(index_buffers(ctx, t, G, C));
+        FTRY(begin_table(ctx, t, req, &tm));
         j->front_cap = 0;
     }
     int64_t cap = j->front_cap;
@@ -2406,17 +2391,14 @@ static int front_chunked(scde_b200_ctx *ctx, scde_b200_diff_job *j, int phase, b
             const int64_t have = (int64_t)(t.q.cap / (size_t)q_row_bytes(t.K));  // a workspace from an earlier call
             if (have > cap) cap = have;
             if (cap > 0x7fffffff) cap = 0x7fffffff;
-            FTRY(reserve_rows(t, pl, (size_t)cap));
+            FTRY(reserve_rows(t, (size_t)cap));
             FCUDA(t.row_x.ensure((size_t)cap));
             j->front_cap = cap;
         }
         FCUDA(launch_dedup_emit(cnt, G, 0, G, n, t.row_off.p + c0, t.row_x.p, t.ridx.p + c0, t.ld_ridx, t.err.p, cap, bits,
                                 st));
         tm.end(SCDE_B200_T_DEDUP, e0, st, 5);
-        e0 = tm.begin(st);
-        int nl = 0;
-        FTRY(launch_table_rows(ctx, t, pl, CellRange{c0, c0 + n, cap}, j->models.m.p, C, j->models.local_theta, &nl));
-        tm.end(SCDE_B200_T_LPTABLE, e0, st, nl);
+        FTRY(table_rows(ctx, t, j->models, CellRange{c0, c0 + n, cap}, &tm));
     }
     tr_queued = since();
     if (trace && last_phase) {
@@ -2438,22 +2420,12 @@ static int front_chunked(scde_b200_ctx *ctx, scde_b200_diff_job *j, int phase, b
     if (trace)
         fprintf(stderr, "[scde_b200] front%s: first chunk counted %.2f ms, chunks queued %.2f, copies done %.2f, draws staged (incl. wait) %.2f, done %.2f\n",
                 !split ? "" : (phase == 0 ? " (first group's chunks)" : " (rest)"), tr_first, tr_queued, tr_copy, tr_draws, tr_front);
+    FTRY(dedup_error(err));
 #undef FTRY
 #undef FCUDA
-    if (err & 1) {
-        cudaStreamSynchronize(ctx->copy_stream);
-        set_error("negative count in the count matrix");
-        return SCDE_B200_EINVAL;
-    }
-    if (err & 2) {
-        cudaStreamSynchronize(ctx->copy_stream);
-        set_error("a cell has >= 32768 distinct count values among the processed genes (hash capacity)");
-        return SCDE_B200_ELIMIT;
-    }
     if (total < 0 || (int64_t)total > cap) return SCDE_B200_OK;  // more rows than estimated: classic rebuild
     t.n_rows = total;
-    t.has_q = true;
-    t.f64_rows = false;
+    if (last_phase) TRY(finish_table(ctx, t, &tm));
     *done = true;
     return SCDE_B200_OK;
 }
@@ -2465,7 +2437,7 @@ extern "C" {
 int scde_b200_diff_upload(scde_b200_ctx *ctx, const scde_b200_diff_args *a, int32_t want_posteriors,
                           scde_b200_diff_job **out) {
     CHECK_CTX(ctx);
-    return diff_upload_impl(ctx, contraction_choice(ctx), a, want_posteriors, out, false);
+    return diff_upload_impl(ctx, a, want_posteriors, out, false);
 }
 
 int scde_b200_diff_run(scde_b200_ctx *ctx, scde_b200_diff_job *j) {
@@ -2484,8 +2456,7 @@ static int diff_run_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, bool chunked
     SCDE_CUDA(j->ws->scr.total.ensure(5));
     SCDE_CUDA(cudaMemsetAsync(j->ws->scr.total.p, 0, 5 * sizeof(unsigned long long), st));
     const int G = j->G, C = j->C, K = j->K;
-    const int ld = j->ws->table.ld;
-    j->ws->table.want_q = k.kernel == Contraction::I8;
+    const int ld = table_ld(K);
     SCDE_CUDA(cudaMemsetAsync(j->status.p, 0, 3 * sizeof(int32_t), st));
     int t_all = tm.begin(st);
     bool front_done = false, joint0_done = false;
@@ -2496,13 +2467,13 @@ static int diff_run_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, bool chunked
                          ld, j->ws->scr, j->status.p + i, &tm, true);
     };
     if (chunked_counts) {
-        TRY(front_chunked(ctx, j, 0, &front_done));
+        TRY(front_chunked(ctx, j, k, 0, &front_done));
         if (front_done && j->split_chunks > 0 && j->split_chunks < j->copy_chunks) {
             // split front: every row of the first group's cells is built and within the capacity -- its joint runs
             // while the rest of the count matrix is still arriving
             TRY(group_joint(0));
             joint0_done = true;
-            TRY(front_chunked(ctx, j, 1, &front_done));
+            TRY(front_chunked(ctx, j, k, 1, &front_done));
             if (!front_done) {  // the table is rebuilt below: row ids change, the first joint is repeated
                 joint0_done = false;
                 SCDE_CUDA(cudaMemsetAsync(j->ws->scr.total.p, 0, 5 * sizeof(unsigned long long), st));
@@ -2521,7 +2492,7 @@ static int diff_run_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, bool chunked
         const int64_t known = (!chunked_counts && k.kernel == Contraction::I8) ? j->known_rows : 0;
         TRY(index_from_counts(ctx, j->ws->table, j->ws->counts.p, G, 0, G, C, &tm, known));
         j->rows_unchecked = known > 0;
-        TRY(fill_rows(ctx, j->ws->table, j->models, j->mag.p, &tm));
+        TRY(fill_table(ctx, j->ws->table, diff_table(j->models, j->mag.p, K, k), &tm));
     }
     for (int i = 0; i < 2; ++i)
         if (!(i == 0 && joint0_done)) TRY(group_joint(i));
@@ -2529,7 +2500,7 @@ static int diff_run_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, bool chunked
     if (j->has_batch) {
         // batch.models differ from models: the table rows are rebuilt from them (same row ids -- the counts have not
         // changed -- so the index matrix stays); the group joints above are done with the first table
-        if (j->bmodels.m.p) TRY(fill_rows(ctx, j->ws->table, j->bmodels, j->mag.p, &tm));
+        if (j->bmodels.m.p) TRY(fill_table(ctx, j->ws->table, diff_table(j->bmodels, j->mag.p, K, k), &tm));
         // the two composition-sampled joints walk the same cells and rows with different draws: one launch of the contraction
         // kernel for both, items paired on neighbouring SMs, so the table is pulled from DRAM once for the two
         const Joint batch[2] = {{j->boot_ptr[2], j->D[2], j->ws->jp[2].p}, {j->boot_ptr[3], j->D[3], j->ws->jp[3].p}};
@@ -2666,7 +2637,7 @@ static int expression_difference_single(scde_b200_ctx *ctx, const scde_b200_diff
     };
     const auto t0 = now();
     scde_b200_diff_job *job = nullptr;
-    int r = diff_upload_impl(ctx, k, args, want_post, &job, true);
+    int r = diff_upload_impl(ctx, args, want_post, &job, true);
     if (r != SCDE_B200_OK) return r;
     const auto t1 = now();
     r = diff_run_impl(ctx, job, true, k);
@@ -2792,9 +2763,8 @@ int ensure_rows(DatasetShard &sh, int from_batch, ContractChoice k, StageTimer *
     LpTable &t = sh.ws->table;
     const bool i8 = k.kernel == Contraction::I8;
     if (sh.rows_from == from_batch && sh.rows_i8 == i8 && !from_batch) return SCDE_B200_OK;
-    t.want_q = i8;
     sh.rows_from = -1;  // unknown until the rebuild has been queued
-    TRY(fill_rows(ctx, t, from_batch ? sh.bmodels : sh.models, sh.mag.p, tm));
+    TRY(fill_table(ctx, t, diff_table(from_batch ? sh.bmodels : sh.models, sh.mag.p, sh.K, k), tm));
     sh.rows_from = from_batch;
     sh.rows_i8 = i8;
     return SCDE_B200_OK;
@@ -2822,15 +2792,15 @@ int shard_create(scde_b200_ctx *ctx, const scde_b200_dataset_args *a, int g0, in
         const std::vector<double> mag = grid_magnitudes(a->prior_x, K);
         TRY(upload(sh->mag, mag.data(), (size_t)K, st));
         LpTable &t = sh->ws->table;
-        init_table(ctx, contraction_choice(ctx), t, K, C, sh->models.fast_theta);
+        const ContractChoice k = contraction_choice(ctx);
         StageTimer &tm = sh->timer;
         tm.reset();
         const int t_all = tm.begin(st);
         TRY(index_from_counts(ctx, t, sh->ws->counts.p, G, 0, G, C, &tm));
-        TRY(fill_rows(ctx, t, sh->models, sh->mag.p, &tm));
+        TRY(fill_table(ctx, t, diff_table(sh->models, sh->mag.p, K, k), &tm));
         tm.end(SCDE_B200_T_TOTAL, t_all, st, 0);
         sh->rows_from = 0;
-        sh->rows_i8 = t.want_q;
+        sh->rows_i8 = k.kernel == Contraction::I8;
         SCDE_CUDA(cudaStreamSynchronize(st));
         return SCDE_B200_OK;
     };

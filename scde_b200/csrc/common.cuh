@@ -56,23 +56,41 @@ cudaError_t launch_based_flags(const double *table, int ld_table, int K, double 
 // zero_compact_c0 >= 0: the FP64 table is the COMPACT one -- one row per cell, its zero-count row, at the cell's index --
 // and zero_row / based point at cell zero_compact_c0 (the fused fixed-point path stores no other FP64 row, so the table is
 // n_cells rows instead of one per distinct (cell, count): 33 MB instead of 40 GB at config 4)
-// One warp per table row.  Writes table[r*ld_table + k] (k >= K zero-filled up to ld_table) and row_mode[r] (first
-// argmax, before the clamp).  which: 0 = every row, plain values; 1 = only the zero-count rows (plain values);
-// 2 = every row except the zero-count ones, stored as the difference to the cell's zero-count row when based[cell].
-cudaError_t launch_lp_rows(const double *models, int ld_models, CellRange cr, const int32_t *row_off,
-                           const int32_t *row_cell_map, const int32_t *row_x, CellPrep prep, int K,
-                           int local_theta, double sentinel, double *table, int ld_table, int32_t *row_mode, int which,
-                           const int32_t *zero_row, const int32_t *based, void *row_const, const int32_t *row_snap,
-                           int write_f64, int8_t *qtable, uint32_t *row_range, cudaStream_t st, int legacy_q_rows = 0,
-                           unsigned long long *work_counter = nullptr, int zero_compact = 0, int8_t *qbound = nullptr);
-// legacy_q_rows: build fixed-point-only rows with the per-element kernel the register-resident one replaced (tests)
-// work_counter: one device word the register-resident row kernel hands its row chunks out from (zeroed by the launcher;
-// required whenever that kernel is chosen, i.e. qtable != NULL with which == 2 on the constant-theta path)
-// zero_compact: `table` is the compact FP64 table (see launch_based_flags); which == 1 writes a cell's zero-count row at the
-// cell's index, which == 2 reads it there
-// write_f64 = 0: the FP64 row is not stored (table is still read for the zero-count rows); qtable != NULL: also emit the
-// row's fixed-point planes and its non-sentinel range (contract_i8.cu) -- both only on the constant-theta fast path -- and,
-// when qbound != NULL, its bound row (Q_BW bytes per row)
+// What every row launch of a table shares.  A row is written as table[r*ld_table + k] (k >= K zero-filled up to ld_table),
+// and row_mode[r] (first argmax, before the clamp) where a launcher takes row_mode != NULL.
+struct RowArgs {
+    const double *models;  // n_cells x 12 column-major with leading dimension ld_models
+    int ld_models;
+    const int32_t *row_off, *row_cell, *row_x;
+    CellPrep prep;
+    int K;
+    double sentinel;
+    double *table;
+    int ld_table;
+    bool fast;  // the constant-theta kernels (K <= KP_TILED, no local theta) on launch_row_consts' output, else the general one
+    const void *row_const;
+    const int32_t *row_snap;
+    int local_theta;
+    const int32_t *zero_row, *based;  // zero-base form: each cell's zero-count row, and whether it can be subtracted
+    bool compact;  // the compact FP64 table (launch_based_flags): zero-count rows at their cell's index, the rest in fixed point
+};
+// The fixed-point planes and non-sentinel range of every row written (contract_i8.cu), and its bound row (Q_BW bytes per
+// row) when bound != NULL.  Constant-theta kernels only.
+struct RowPlanes {
+    int8_t *q;
+    uint32_t *range;
+    int8_t *bound;
+};
+// One warp per row.  The zero-count rows of the cells of cr (plain values), with their planes when q.q != NULL.
+cudaError_t launch_zero_count_rows(const RowArgs &a, CellRange cr, int32_t *row_mode, RowPlanes q, cudaStream_t st);
+// The other rows of cr, as the difference to the cell's zero-count row where based[cell].  q.q != NULL: planes only (the
+// per-element form of launch_q_rows); otherwise FP64 rows.
+cudaError_t launch_nonzero_rows(const RowArgs &a, CellRange cr, int32_t *row_mode, RowPlanes q, cudaStream_t st);
+// Every row of cr, plain values, FP64 only.
+cudaError_t launch_dense_rows(const RowArgs &a, CellRange cr, int32_t *row_mode, cudaStream_t st);
+// The rows of non-zero counts of cr in fixed point only, on the register-resident kernel (constant-theta, compact table);
+// it hands out its row chunks from the device word *work_counter, which the launcher zeroes.
+cudaError_t launch_q_rows(const RowArgs &a, CellRange cr, RowPlanes q, unsigned long long *work_counter, cudaStream_t st);
 // per-row constants of the constant-theta fast path (4 doubles per row), one thread per row
 // ... and row_snap[r] = grid point where the reference's snap rule replaces mu_k by the count, or -1 (needs prep.mu)
 cudaError_t launch_row_consts(const double *models, int ld_models, const int32_t *row_off, CellRange cr,

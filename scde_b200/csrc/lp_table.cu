@@ -1172,66 +1172,75 @@ cudaError_t launch_based_flags(const double *table, int ld_table, int K, double 
     return cudaGetLastError();
 }
 
-cudaError_t launch_lp_rows(const double *models, int ld_models, CellRange cr, const int32_t *row_off,
-                           const int32_t *row_cell_map, const int32_t *row_x, CellPrep prep, int K,
-                           int local_theta, double sentinel, double *table, int ld_table, int32_t *row_mode, int which,
-                           const int32_t *zero_row, const int32_t *based, void *row_const, const int32_t *row_snap,
-                           int write_f64, int8_t *qtable, uint32_t *row_range, cudaStream_t st, int legacy_q_rows,
-                           unsigned long long *work_counter, int zero_compact, int8_t *qbound) {
+namespace {
+
+// The row kernels of the table take their rows' bounds on the device: the grid is sized for the cells (hundreds of rows
+// each) and strides over the rows.  which: 0 every row, 1 the zero-count rows, 2 the others.
+cudaError_t launch_row_kernel(const RowArgs &a, CellRange cr, int which, int32_t *row_mode, const int32_t *zero_row,
+                              const int32_t *based, int write_f64, RowPlanes q, cudaStream_t st) {
     if (cr.c1 <= cr.c0) return cudaSuccess;
-    // compact FP64 table (one row per cell: its zero-count row): only the zero-count rows may be stored in FP64
-    if (zero_compact && (which == 0 || (which == 2 && write_f64) || local_theta)) return cudaErrorInvalidValue;
-    // the number of rows is only known on the device: size the grid for the cells (hundreds of rows each), grid-stride
     int64_t blocks = which == 1 ? ((int64_t)(cr.c1 - cr.c0) + ROW_WARPS - 1) / ROW_WARPS : (int64_t)(cr.c1 - cr.c0) * 8;
     const int64_t cap = 148 * 64;
     if (blocks > cap) blocks = cap;
-    if (qtable && (!row_range || K > Q_MAX_K)) return cudaErrorInvalidValue;
-    if (prep.cfp && prep.scfp && row_const && !local_theta && K <= KP_TILED && ld_table >= round_up(K, 16)) {
-        if (!row_snap) return cudaErrorInvalidValue;
-        if (which == 2 && qtable && !write_f64 && !row_mode && zero_row && based && prep.ld >= K && !legacy_q_rows) {
-            // fixed-point rows only: the register-resident kernel; one contiguous run of rows per warp
-            const size_t smem = (size_t)QR_WARPS * QR_SMEM_WARP;
-            auto launch_q = [&](auto kernel) -> cudaError_t {
-                cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-                if (e != cudaSuccess) return e;
-                if (!work_counter) return cudaErrorInvalidValue;
-                e = cudaMemsetAsync(work_counter, 0, sizeof(unsigned long long), st);
-                if (e != cudaSuccess) return e;
-                kernel<<<148 * 3, QR_WARPS * 32, smem, st>>>(models, ld_models, cr, row_off, row_cell_map, row_x,
-                                                             (const double4 *)row_const, row_snap, prep, K, sentinel, table,
-                                                             ld_table, zero_row, based, qtable, q_row_bytes(K), row_range,
-                                                             work_counter, zero_compact, qtable ? qbound : nullptr);
-                return cudaGetLastError();
-            };
-            if (qbound)
-                return K >= 4 * 32 * QR_MAIN ? launch_q(lp_rows_q_kernel<true, true>) : launch_q(lp_rows_q_kernel<false, true>);
-            return K >= 4 * 32 * QR_MAIN ? launch_q(lp_rows_q_kernel<true, false>) : launch_q(lp_rows_q_kernel<false, false>);
-        }
-        auto launch =[&](auto kernel, int rpw) -> cudaError_t {
-            const size_t smem = (size_t)ROW_WARPS * rpw * (sizeof(double) * KP_TILED + 4 * Q_PIECE);
+    if (a.fast) {
+        auto launch = [&](auto kernel) -> cudaError_t {
+            const size_t smem = (size_t)ROW_WARPS * 2 * (sizeof(double) * KP_TILED + 4 * Q_PIECE);
             cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
             if (e != cudaSuccess) return e;
             kernel<<<(unsigned)blocks, ROW_WARPS * 32, smem, st>>>(
-                models, ld_models, cr, row_off, row_cell_map, row_x, (const double4 *)row_const, row_snap, prep, K, sentinel,
-                table, ld_table, row_mode, which, zero_row, based, write_f64, zero_compact, qtable, q_row_bytes(K), row_range,
-                qtable ? qbound : nullptr);
+                a.models, a.ld_models, cr, a.row_off, a.row_cell, a.row_x, (const double4 *)a.row_const, a.row_snap, a.prep,
+                a.K, a.sentinel, a.table, a.ld_table, row_mode, which, zero_row, based, write_f64, a.compact, q.q,
+                q_row_bytes(a.K), q.range, q.bound);
             return cudaGetLastError();
         };
-        const bool norm = write_f64 != 0;  // rows that exist in fixed point only need no normalising constant
+        // rows that exist in fixed point only need no normalising constant
         if (row_mode)
-            return norm ? launch(lp_rows_fast_kernel<true, 16, true>, 2) : launch(lp_rows_fast_kernel<true, 16, false>, 2);
-        return norm ? launch(lp_rows_fast_kernel<false, 16, true>, 2) : launch(lp_rows_fast_kernel<false, 16, false>, 2);
+            return write_f64 ? launch(lp_rows_fast_kernel<true, 16, true>) : launch(lp_rows_fast_kernel<true, 16, false>);
+        return write_f64 ? launch(lp_rows_fast_kernel<false, 16, true>) : launch(lp_rows_fast_kernel<false, 16, false>);
     }
-    if (qtable || !write_f64) return cudaErrorInvalidValue;  // the general kernel writes the FP64 table only
-    size_t smem = (size_t)ROW_WARPS * K * sizeof(double);
+    size_t smem = (size_t)ROW_WARPS * a.K * sizeof(double);
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(lp_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
     }
-    lp_rows_kernel<<<(unsigned)blocks, ROW_WARPS * 32, smem, st>>>(models, ld_models, cr, row_off, row_cell_map, row_x, prep, K,
-                                                                  local_theta, sentinel, table, ld_table, row_mode, which,
-                                                                  zero_row, based);
+    lp_rows_kernel<<<(unsigned)blocks, ROW_WARPS * 32, smem, st>>>(a.models, a.ld_models, cr, a.row_off, a.row_cell, a.row_x,
+                                                                    a.prep, a.K, a.local_theta, a.sentinel, a.table, a.ld_table,
+                                                                    row_mode, which, zero_row, based);
     return cudaGetLastError();
+}
+
+}  // namespace
+
+cudaError_t launch_zero_count_rows(const RowArgs &a, CellRange cr, int32_t *row_mode, RowPlanes q, cudaStream_t st) {
+    return launch_row_kernel(a, cr, 1, row_mode, a.zero_row, nullptr, 1, q, st);
+}
+
+cudaError_t launch_nonzero_rows(const RowArgs &a, CellRange cr, int32_t *row_mode, RowPlanes q, cudaStream_t st) {
+    return launch_row_kernel(a, cr, 2, row_mode, a.zero_row, a.based, q.q ? 0 : 1, q, st);
+}
+
+cudaError_t launch_dense_rows(const RowArgs &a, CellRange cr, int32_t *row_mode, cudaStream_t st) {
+    return launch_row_kernel(a, cr, 0, row_mode, nullptr, nullptr, 1, RowPlanes{}, st);
+}
+
+cudaError_t launch_q_rows(const RowArgs &a, CellRange cr, RowPlanes q, unsigned long long *work_counter, cudaStream_t st) {
+    if (cr.c1 <= cr.c0) return cudaSuccess;
+    // one contiguous run of rows per warp, handed out from *work_counter
+    const size_t smem = (size_t)QR_WARPS * QR_SMEM_WARP;
+    auto launch = [&](auto kernel) -> cudaError_t {
+        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+        e = cudaMemsetAsync(work_counter, 0, sizeof(unsigned long long), st);
+        if (e != cudaSuccess) return e;
+        kernel<<<148 * 3, QR_WARPS * 32, smem, st>>>(a.models, a.ld_models, cr, a.row_off, a.row_cell, a.row_x,
+                                                       (const double4 *)a.row_const, a.row_snap, a.prep, a.K, a.sentinel,
+                                                       a.table, a.ld_table, a.zero_row, a.based, q.q, q_row_bytes(a.K), q.range,
+                                                       work_counter, a.compact, q.bound);
+        return cudaGetLastError();
+    };
+    const bool full = a.K >= 4 * 32 * QR_MAIN;
+    if (q.bound) return full ? launch(lp_rows_q_kernel<true, true>) : launch(lp_rows_q_kernel<false, true>);
+    return full ? launch(lp_rows_q_kernel<true, false>) : launch(lp_rows_q_kernel<false, false>);
 }
 
 }  // namespace scde
