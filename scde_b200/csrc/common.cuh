@@ -203,7 +203,7 @@ inline int q_pieces(int K) { return (K + Q_PW - 1) / Q_PW; }
 // Bound rows (DESIGN.md 4.3, "Pruned pieces"): next to its planes every fixed-point row has Q_BW bytes of bounds on its value
 // x = 2^29 D, in units of 2^-5 nat (x / 2^24), rounded outwards: slot u < Q_UB_N holds ceil(max x / 2^24) over the row's
 // non-sentinel points of grid block [16 u, 16 u + 16) (0 when it has none), slot Q_UB_N + c floor(x / 2^24) at the sample
-// point Q_LB_STEP c + Q_LB_OFF (0 at a sentinel).  Slot i is stored as two signed radix-256 digits, bytes i and
+// point Q_LB_STEP c + Q_LB_OFF (0 at a sentinel or beyond the grid), every later slot 0.  Slot i is stored as two signed radix-256 digits, bytes i and
 // Q_BSLOTS + i, so that the contraction over the drawn rows (the tcgen05 kernel with one 128-byte piece) sums them exactly.
 constexpr int Q_BW = 128;
 constexpr int Q_BSLOTS = Q_BW / 2;
@@ -244,6 +244,8 @@ __device__ inline void q_bound_row(const int8_t *q, int K, uint32_t range, int8_
         const int k = Q_LB_STEP * c + Q_LB_OFF;
         q_bound_store(brow, Q_UB_N + c, k < K ? (int)(q_value_at(q, k) >> 24) : 0);
     }
+    // the unused slots: the row buffer is not cleared when it is allocated
+    for (int s = Q_UB_N + Q_LB_N + l; s < Q_BSLOTS; s += LW) q_bound_store(brow, s, 0);
 }
 #endif
 // planes and ranges of every row of an FP64 table (ld_table >= K); one warp per row

@@ -19,7 +19,8 @@ def _decision(qb, rr, W, Z, lists, K):
     G = len(lists)
     zb = np.full((WP, 64), -np.inf)
     for u in range(UB_N):
-        zb[:, u] = Z[:, u * UB_PTS:min((u + 1) * UB_PTS, K)].max(axis=1)
+        if u * UB_PTS < K:  # (blocks past the grid keep -inf, as z_bounds_kernel writes them)
+            zb[:, u] = Z[:, u * UB_PTS:min((u + 1) * UB_PTS, K)].max(axis=1)
     for c in range(LB_N):
         if LB_STEP * c + LB_OFF < K:
             zb[:, UB_N + c] = Z[:, LB_STEP * c + LB_OFF]

@@ -151,26 +151,34 @@ Q_PW, Q_PIECE, UB_PTS, UB_N, LB_STEP, LB_OFF, LB_N = 102, 512, 16, 26, 12, 6, 35
 WP, KP = 104, 416
 
 
-def _table(ctx, n_genes, n_cells, seed):
-    """the fused table of a config-4-like workload, with its bound rows (scde_b200_probe_table_bounds)"""
-    w = synth.make_workload(4, n_genes=n_genes, n_cells=n_cells, seed=seed)
-    counts = np.asarray(w.counts, dtype=np.int32)
-    mm, lt, sq = api.pack_models(w.models)
+def _table(ctx, n_genes, n_cells, seed, K=None, inputs=None, **options):
+    """the fused table of a config-4-like workload -- or of inputs = (models, counts) -- on the prior's grid or on one of K
+    points, with its bound rows (scde_b200_probe_table_bounds), under the given scde_b200_options fields"""
+    if inputs is None:
+        w = synth.make_workload(4, n_genes=n_genes, n_cells=n_cells, seed=seed)
+        inputs = w.models, w.counts
+    counts = np.asarray(inputs[1], dtype=np.int32)
+    n_cells = counts.shape[1]
+    mm, lt, sq = api.pack_models(inputs[0])
     mm = np.asfortranarray(mm, dtype=np.float64)
-    x = w.prior["x"].to_numpy()
+    x = synth.make_prior(n_genes, length_out=(K or 401) - 1)["x"].to_numpy()
     K = len(x)
     with np.errstate(divide="ignore"):
         mag = np.log(np.maximum(10.0 ** x - 1.0, 0.0))
     flat, off, uci = api._unique_index(counts)
     n_rows = int(off[-1])
-    out = dict(q=np.zeros((n_rows, 4 * Q_PIECE), np.int8), rr=np.zeros(n_rows, np.uint32),
+    out = dict(q=np.zeros((n_rows, -(-K // Q_PW) * Q_PIECE), np.int8), rr=np.zeros(n_rows, np.uint32),
                zero_row=np.empty(n_cells, np.int32), based=np.empty(n_cells, np.int32), zero_rows=np.empty((n_cells, K)),
-               qb=np.zeros((n_rows, 128), np.int8))
+               qb=np.full((n_rows, 128), 0x55, np.int8))  # (not a bound row: a row the probe leaves unwritten shows)
     vp = lambda a: a.ctypes.data_as(C.c_void_p)
-    _lib.check(_lib.lib().scde_b200_probe_table_bounds(
-        ctx.handle, _lib.p_f64(mm), n_cells, _lib.p_i32(np.ascontiguousarray(flat, np.int32)), _lib.p_i32(off),
-        _lib.p_f64(np.ascontiguousarray(mag)), K, lt, sq, n_cells, vp(out["q"]), vp(out["rr"]), _lib.p_i32(out["zero_row"]),
-        _lib.p_i32(out["based"]), _lib.p_f64(out["zero_rows"]), vp(out["qb"])))
+    keep = ctx.set_options(**options)
+    try:
+        _lib.check(_lib.lib().scde_b200_probe_table_bounds(
+            ctx.handle, _lib.p_f64(mm), n_cells, _lib.p_i32(np.ascontiguousarray(flat, np.int32)), _lib.p_i32(off),
+            _lib.p_f64(np.ascontiguousarray(mag)), K, lt, sq, n_cells, vp(out["q"]), vp(out["rr"]),
+            _lib.p_i32(out["zero_row"]), _lib.p_i32(out["based"]), _lib.p_f64(out["zero_rows"]), vp(out["qb"])))
+    finally:
+        ctx.restore_options(keep)
     out.update(counts=counts, off=off, uci=uci, K=K)
     return out
 

@@ -391,23 +391,49 @@ def test_sentinel_zero_row_model_is_not_based():
 
 
 # ---- GPU: the probe against the oracle -----------------------------------------------------------------------------------
-def probe(ctx, case, **options):
-    """scde_b200_probe_table under the given scde_b200_options fields"""
+def probe(ctx, case, bounds=False, **options):
+    """scde_b200_probe_table under the given scde_b200_options fields; bounds: scde_b200_probe_table_bounds, with the
+    bound rows in out["qb"]"""
     n_rows, K = int(case.off[-1]), case.K
     out = {"q": np.zeros((n_rows, q_row_bytes(K)), np.int8), "range": np.zeros(n_rows, np.uint32),
            "zero_row": np.empty(case.n_cells, np.int32), "based": np.empty(case.n_cells, np.int32),
            "zero_rows": np.empty((case.n_cells, K))}
-    keep = ctx.set_options(**options)
-    try:
-        _lib.check(_lib.lib().scde_b200_probe_table(
-            ctx.handle, _lib.p_f64(case.mm), case.n_cells, _lib.p_i32(case.flat), _lib.p_i32(case.off),
+    args = [ctx.handle, _lib.p_f64(case.mm), case.n_cells, _lib.p_i32(case.flat), _lib.p_i32(case.off),
             _lib.p_f64(_lib.f64(case.mag)), K, case.lt, case.sq, case.clamp, out["q"].ctypes.data_as(C.c_void_p),
             out["range"].ctypes.data_as(C.c_void_p), _lib.p_i32(out["zero_row"]), _lib.p_i32(out["based"]),
-            _lib.p_f64(out["zero_rows"])))
+            _lib.p_f64(out["zero_rows"])]
+    if bounds:
+        out["qb"] = np.full((n_rows, 128), 0x55, np.int8)  # (not a bound row: a row the probe leaves unwritten shows)
+        args.append(out["qb"].ctypes.data_as(C.c_void_p))
+    keep = ctx.set_options(**options)
+    try:
+        fn = _lib.lib().scde_b200_probe_table_bounds if bounds else _lib.lib().scde_b200_probe_table
+        _lib.check(fn(*args))
     finally:
         ctx.restore_options(keep)
     out["X"] = decode(out["q"], K)
     return out
+
+
+def row_reference(case, out, c, j):
+    """the oracle's values of row j of cell c as the planes of the probe hold them, for a row with a regular range:
+    (want, normal, both, c_row) -- want = lp - Z (Z = the cell's zero-count row where the row is stored as the difference
+    to it), the elements whose lp and Z are above -700, the elements that are "log 0" on neither side, and the row
+    constant c_row the planes add (fused rows omit log S): the median of planes - want over the normal elements both
+    sides hold, 0 when there are none.  The planes' value of an element is want + c_row."""
+    K = case.K
+    k = np.arange(K)
+    x, lp = case.lists[c][j], case.ref[c][:, j]
+    z_dev = out["zero_rows"][c]
+    sub = bool(out["based"][c]) and x != 0
+    want = lp - (z_dev if sub else 0.0)
+    normal = (lp > -700.0) & ((z_dev > -700.0) if sub else True)
+    rr = int(out["range"][case.off[c] + j])
+    both = (lp > LOG0) & (k >= (rr & 0xFFFF)) & (k <= rr >> 16)
+    v = out["X"][case.off[c] + j] / SCALE
+    sel = both & normal if np.any(both & normal) else both
+    c_row = float(np.median(v[sel] - want[sel])) if np.any(sel) else 0.0
+    return want, normal, both, c_row
 
 
 def check_probe(case, out):
@@ -434,8 +460,6 @@ def check_probe(case, out):
             lp = ref[:, j]
             sub = based and x != 0
             Z = z_dev if sub else np.zeros(K)
-            want = lp - Z
-            normal = (lp > -700.0) & ((z_dev > -700.0) if sub else True)
             X, rr = out["X"][r], int(out["range"][r])
             where = f"cell {c} count {x} (row {r}, based {based})"
             ref_ok = lp > LOG0
@@ -451,10 +475,8 @@ def check_probe(case, out):
             dev_ok = (k >= lo) & (k <= hi)
             assert np.all(X[~dev_ok] == 0), f"{where}: digits of a \"log 0\" element"
             seen["log0"] += int(np.sum(~dev_ok))
-            both = ref_ok & dev_ok
+            want, normal, both, c_row = row_reference(case, out, c, j)
             v = X / SCALE
-            sel = both & normal if np.any(both & normal) else both
-            c_row = float(np.median(v[sel] - want[sel])) if np.any(sel) else 0.0
             flip = ref_ok != dev_ok
             if flip.any():
                 seen["flips"] += int(flip.sum())
