@@ -74,8 +74,8 @@ struct RowArgs {
     const int32_t *zero_row, *based;  // zero-base form: each cell's zero-count row, and whether it can be subtracted
     bool compact;  // the compact FP64 table (launch_based_flags): zero-count rows at their cell's index, the rest in fixed point
 };
-// The fixed-point planes and non-sentinel range of every row written (contract_i8.cu), and its bound row (Q_BW bytes per
-// row) when bound != NULL.  Constant-theta kernels only.
+// The fixed-point planes and non-sentinel range of every row written (the fixed-point form, described below), and its
+// bound row (Q_BW bytes per row) when bound != NULL.  Constant-theta kernels only.
 struct RowPlanes {
     int8_t *q;
     uint32_t *range;
@@ -96,6 +96,9 @@ cudaError_t launch_q_rows(const RowArgs &a, CellRange cr, RowPlanes q, unsigned 
 cudaError_t launch_row_consts(const double *models, int ld_models, const int32_t *row_off, CellRange cr,
                               const int32_t *row_cell, const int32_t *row_x, void *row_const, int32_t *row_snap,
                               CellPrep prep, int K, cudaStream_t st);
+// planes, ranges and bound rows (qbound != NULL) of every row of an FP64 table (K <= ld_table, a multiple of 4)
+cudaError_t launch_quantize_rows(const double *table, int ld_table, int K, int64_t n_rows, int8_t *qtable,
+                                 uint32_t *row_range, int8_t *qbound, cudaStream_t st);
 
 // ---- dedup.cu ------------------------------------------------------------------------------------
 // counts: column-major with leading dimension ld_counts; genes [g0, g0+G) of n_cells columns.
@@ -191,7 +194,8 @@ int contract_tiled_max_genes();  // genes per launch of a tiled kernel (bounds t
 // plane: every row carries the range [klo, khi] of its grid points that are NOT the sentinel (they form one interval for
 // every row the error models produce; a row where they do not is marked Q_RANGE_IRREGULAR and sends the call to the FP64
 // kernel), and a grid point of a (gene, boot) is "log 0" exactly when it lies outside the intersection of the ranges
-// of the drawn rows (sentinel_range_kernel).
+// of the drawn rows (sentinel_range_kernel).  The table's row kernels and the quantize pass (lp_table.cu) write this
+// form, with its bound rows; the contraction reads it.
 constexpr int Q_NV = 5;           // value planes
 constexpr int Q_FRAC = 29;        // fractional bits (|value| <= 1000 < 2^10 fits 5 digits)
 constexpr int Q_PW = 102;         // grid points per piece: Q_NV * Q_PW = 510 of the 512 tensor-memory columns
@@ -217,40 +221,6 @@ __host__ __device__ inline void q_bound_store(int8_t *brow, int slot, int v) {
     brow[Q_BSLOTS + slot] = (int8_t)((v - lo) >> 8);
 }
 inline int q_row_bytes(int K) { return q_pieces(K) * Q_PIECE; }
-#ifdef __CUDACC__
-// the bound row of a fixed-point row from its planes (q: [piece][plane][102], generic address) and its non-sentinel range;
-// lanes l, l + LW, .. of a group of LW lanes take the slots.  (The register-resident row kernel computes the same values
-// from its registers: lp_table.cu.)
-__device__ inline long long q_value_at(const int8_t *q, int k) {
-    const int pc = k / Q_PW, i = k - pc * Q_PW;
-    long long x = 0;
-#pragma unroll
-    for (int pl = Q_NV - 1; pl >= 0; --pl) x = x * 256 + q[pc * Q_PIECE + pl * Q_PW + i];
-    return x;
-}
-__device__ inline void q_bound_row(const int8_t *q, int K, uint32_t range, int8_t *brow, int l, int LW) {
-    int klo = 0, khi = K - 1;
-    if (range != Q_RANGE_IRREGULAR) {
-        klo = (int)(range & 0xFFFFu);
-        khi = (int)(range >> 16);
-    }
-    for (int u = l; u < Q_UB_N; u += LW) {
-        long long m = INT64_MIN;
-        for (int k = max(u * Q_UB_PTS, klo); k < (u + 1) * Q_UB_PTS && k <= khi; ++k) m = max(m, q_value_at(q, k));
-        // ceil(x / 2^24) by an arithmetic shift
-        q_bound_store(brow, u, m == INT64_MIN ? 0 : (int)((m + ((1ll << 24) - 1)) >> 24));
-    }
-    for (int c = l; c < Q_LB_N; c += LW) {
-        const int k = Q_LB_STEP * c + Q_LB_OFF;
-        q_bound_store(brow, Q_UB_N + c, k < K ? (int)(q_value_at(q, k) >> 24) : 0);
-    }
-    // the unused slots: the row buffer is not cleared when it is allocated
-    for (int s = Q_UB_N + Q_LB_N + l; s < Q_BSLOTS; s += LW) q_bound_store(brow, s, 0);
-}
-#endif
-// planes and ranges of every row of an FP64 table (ld_table >= K); one warp per row
-cudaError_t launch_quantize_rows(const double *table, int ld_table, int K, int64_t n_rows, int8_t *qtable,
-                                 uint32_t *row_range, int8_t *qbound, cudaStream_t st);
 // W8[pass][row][128] = (int8) W[pass][row][0..104); *flag |= 1 if a multiplicity exceeds 127
 cudaError_t launch_w_to_i8(const double *W, int n_w_rows, int n_boot, int8_t *W8, int32_t *flag, cudaStream_t st);
 // What the sides of a launch share (see I8Side)

@@ -1075,55 +1075,6 @@ __global__ void exp_probe_kernel(double *out) {
     if (i < 3) out[i] = exp_nonpos(-745.0 - i);
 }
 
-// ------------------------------------------------------------------------------------------------
-// fixed-point planes and non-sentinel range of every row of an FP64 table (the general row kernel writes FP64 only; the
-// constant-theta fast kernel emits both itself, lp_table.cu): one warp per row
-__global__ void __launch_bounds__(256) quantize_rows_kernel(const double *__restrict__ table, int ld_table, int K, int64_t n_rows,
-                                                            int8_t *__restrict__ qtable, int64_t ldq,
-                                                            uint32_t *__restrict__ row_range, int8_t *__restrict__ qbound) {
-    const int64_t row = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    if (row >= n_rows) return;
-    const int lane = threadIdx.x & 31;
-    const double *src = table + row * ld_table;
-    int8_t *dst = qtable + row * ldq;
-    for (int64_t j = lane; j < ldq / 4; j += 32) reinterpret_cast<uint32_t *>(dst)[j] = 0u;
-    __syncwarp();
-    int n_ok = 0, kmin = 0x7fffffff, kmax = -1;
-    for (int k = lane; k < K; k += 32) {
-        const double v = src[k];
-        if (!(v > -1.0e290)) continue;  // the "log 0" sentinel (or a difference to it): digits stay zero
-        ++n_ok;
-        kmin = min(kmin, k);
-        kmax = max(kmax, k);
-        long long x = __double2ll_rn(fmin(fmax(v, -1000.0), 1000.0) * (double)(1ll << Q_FRAC));
-        const int pc = k / Q_PW, i = k - pc * Q_PW;
-#pragma unroll
-        for (int pl = 0; pl < Q_NV; ++pl) {
-            const int d = (int)(int8_t)(x & 0xFF);
-            dst[pc * Q_PIECE + pl * Q_PW + i] = (int8_t)d;
-            x = (x - d) >> 8;
-        }
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        n_ok += __shfl_xor_sync(0xffffffffu, n_ok, o);
-        kmin = min(kmin, __shfl_xor_sync(0xffffffffu, kmin, o));
-        kmax = max(kmax, __shfl_xor_sync(0xffffffffu, kmax, o));
-    }
-    uint32_t rr;
-    if (n_ok == 0)
-        rr = Q_RANGE_IRREGULAR;  // a row of sentinels only: let the FP64 kernel deal with it
-    else if (kmax - kmin + 1 != n_ok)
-        rr = Q_RANGE_IRREGULAR;
-    else
-        rr = (uint32_t)kmin | ((uint32_t)kmax << 16);
-    if (lane == 0) row_range[row] = rr;
-    if (qbound) {
-        __syncwarp();  // the planes the other lanes wrote
-        q_bound_row(dst, K, rr, qbound + row * Q_BW, lane, 32);
-    }
-}
-
 // W (FP64 multiplicities, pass-major [pass][n_w_rows][108]) -> int8 rows of 128 bytes; flag |= 1 when a count > 127
 __global__ void w_to_i8_kernel(const double *__restrict__ W, int64_t n_rows_total, int8_t *__restrict__ W8,
                                int32_t *__restrict__ flag) {
@@ -1145,15 +1096,6 @@ __global__ void w_to_i8_kernel(const double *__restrict__ W, int64_t n_rows_tota
 }
 
 }  // namespace
-
-cudaError_t launch_quantize_rows(const double *table, int ld_table, int K, int64_t n_rows, int8_t *qtable,
-                                 uint32_t *row_range, int8_t *qbound, cudaStream_t st) {
-    if (n_rows <= 0) return cudaSuccess;
-    if (K > ld_table || K > Q_MAX_K) return cudaErrorInvalidValue;
-    quantize_rows_kernel<<<(unsigned)((n_rows + 7) / 8), 256, 0, st>>>(table, ld_table, K, n_rows, qtable, q_row_bytes(K),
-                                                                        row_range, qbound);
-    return cudaGetLastError();
-}
 
 cudaError_t launch_w_to_i8(const double *W, int n_w_rows, int n_boot, int8_t *W8, int32_t *flag, cudaStream_t st) {
     const int passes = (n_boot + WP_TILED - 1) / WP_TILED;

@@ -471,6 +471,81 @@ __device__ __forceinline__ int q_offset(int k) {
     return pc * Q_PIECE + (k - pc * Q_PW);
 }
 
+// the bound row of a fixed-point row from its planes (q: [piece][plane][102], generic address) and its non-sentinel range;
+// lanes l, l + LW, .. of a group of LW lanes take the slots.  (lp_rows_q_kernel computes the same values from its
+// registers.)
+__device__ inline long long q_value_at(const int8_t *q, int k) {
+    const int pc = k / Q_PW, i = k - pc * Q_PW;
+    long long x = 0;
+#pragma unroll
+    for (int pl = Q_NV - 1; pl >= 0; --pl) x = x * 256 + q[pc * Q_PIECE + pl * Q_PW + i];
+    return x;
+}
+__device__ inline void q_bound_row(const int8_t *q, int K, uint32_t range, int8_t *brow, int l, int LW) {
+    int klo = 0, khi = K - 1;
+    if (range != Q_RANGE_IRREGULAR) {
+        klo = (int)(range & 0xFFFFu);
+        khi = (int)(range >> 16);
+    }
+    for (int u = l; u < Q_UB_N; u += LW) {
+        long long m = INT64_MIN;
+        for (int k = max(u * Q_UB_PTS, klo); k < (u + 1) * Q_UB_PTS && k <= khi; ++k) m = max(m, q_value_at(q, k));
+        // ceil(x / 2^24) by an arithmetic shift
+        q_bound_store(brow, u, m == INT64_MIN ? 0 : (int)((m + ((1ll << 24) - 1)) >> 24));
+    }
+    for (int c = l; c < Q_LB_N; c += LW) {
+        const int k = Q_LB_STEP * c + Q_LB_OFF;
+        q_bound_store(brow, Q_UB_N + c, k < K ? (int)(q_value_at(q, k) >> 24) : 0);
+    }
+    // the unused slots: the row buffer is not cleared when it is allocated
+    for (int s = Q_UB_N + Q_LB_N + l; s < Q_BSLOTS; s += LW) q_bound_store(brow, s, 0);
+}
+
+// The row writer of lp_rows_fast_kernel and quantize_rows_kernel.  LW lanes stage a fixed-point row in shared memory (sq:
+// 4 Q_PIECE bytes, cleared once, so the two spare bytes of every piece and the pieces beyond the grid stay zero): lane l
+// passes its j-th quad k0 = 4 l + 4 LW j, whose digits are stored and whose points in the grid and not "log 0" set bits
+// 4 j + e of its okmask.  After a __syncwarp, the row, its range and its bound row (qbound != NULL) are stored if valid.
+template <int LW>
+__device__ __forceinline__ void q_stage_quad(uint8_t *sq, int k0, int j, int K, const double (&v)[4], uint32_t &okmask) {
+    uint32_t word[Q_NV], sent;
+    fixed_point_quad(v, word, sent);
+    const int nk = K - k0;  // real grid points in this quad
+    okmask |= (~sent & (nk >= 4 ? 0xFu : nk > 0 ? (1u << nk) - 1u : 0u)) << (4 * j);
+    // pairs (k0, k0 + 1) and (k0 + 2, k0 + 3) never straddle a piece (Q_PW is even): 16-bit stores
+    uint16_t *dst0 = reinterpret_cast<uint16_t *>(sq + q_offset(k0));
+    uint16_t *dst1 = reinterpret_cast<uint16_t *>(sq + q_offset(k0 + 2));
+#pragma unroll
+    for (int p = 0; p < Q_NV; ++p) {
+        dst0[(p * Q_PW) >> 1] = (uint16_t)(word[p] & 0xFFFFu);
+        dst1[(p * Q_PW) >> 1] = (uint16_t)(word[p] >> 16);
+    }
+}
+template <int LW>
+__device__ __forceinline__ void q_store_row(const uint8_t *sq, uint32_t okmask, int l, int K, int64_t row, bool valid,
+                                            int8_t *qtable, int ldq, uint32_t *row_range, int8_t *qbound) {
+    // the row's planes, 16 bytes per lane and store
+    const uint4 *src = reinterpret_cast<const uint4 *>(sq);
+    uint4 *dst = reinterpret_cast<uint4 *>(qtable + (size_t)row * ldq);
+    if (valid)
+        for (int j = l; j < ldq / 16; j += LW) dst[j] = src[j];
+    // count, first and last of the grid points that are not "log 0" (bit b of a lane <-> k = 4 l + 4 LW (b >> 2) + (b & 3))
+    int n_ok = __popc(okmask), kmin = 0x7fffffff, kmax = -1;
+    if (okmask) {
+        const int b0 = __ffs(okmask) - 1, b1 = 31 - __clz(okmask);
+        kmin = 4 * l + 4 * LW * (b0 >> 2) + (b0 & 3);
+        kmax = 4 * l + 4 * LW * (b1 >> 2) + (b1 & 3);
+    }
+#pragma unroll
+    for (int o = LW / 2; o > 0; o >>= 1) {
+        n_ok += __shfl_xor_sync(0xffffffffu, n_ok, o);
+        kmin = min(kmin, __shfl_xor_sync(0xffffffffu, kmin, o));
+        kmax = max(kmax, __shfl_xor_sync(0xffffffffu, kmax, o));
+    }
+    const uint32_t rr = (n_ok > 0 && kmax - kmin + 1 == n_ok) ? ((uint32_t)kmin | ((uint32_t)kmax << 16)) : Q_RANGE_IRREGULAR;
+    if (l == 0 && valid) row_range[row] = rr;
+    if (qbound && valid) q_bound_row(reinterpret_cast<const int8_t *>(sq), K, rr, qbound + (size_t)row * Q_BW, l, LW);
+}
+
 // The sweeps (one warp per row; lane l owns the grid points 4 l + 128 j .. + 3, so every access is a 16- or 32-byte
 // vector and the index arithmetic is shared by four points; the row lives in a per-warp shared-memory buffer):
 //   1. a_k = log NB_k + log(1 - d_k) and its maximum;  M = max(max_k a_k, max_k log d_k + f)          (:188-192)
@@ -490,22 +565,22 @@ __device__ __noinline__ double lp_slow_element(double a, double dk, double lsum,
     return t >= sentinel ? t : sentinel;
 }
 
-// LW lanes per row (32: one row per warp; 16: two rows per warp, side by side in the two half-warps -- 101 quads of a
-// 401-point grid then occupy 7 x 16 = 112 lane slots instead of 4 x 32 = 128, every warp shuffle of the reductions serves
-// two rows, and twice as many independent rows are in flight per warp).
+// LW = 16 lanes per row: two rows per warp, side by side in the two half-warps -- 101 quads of a 401-point grid then
+// occupy 7 x 16 = 112 lane slots instead of 4 x 32 = 128, every warp shuffle of the reductions serves two rows, and twice
+// as many independent rows are in flight per warp.
 // NORM = false: the row is stored without its normalising constant log S (sweep 2 is skipped).  A constant added to a
 // whole table row adds a constant to T[b, :] of every (gene, boot) that draws the row, which the soft-max over the grid
 // removes: the joint posterior cannot see it.  Only the fixed-point rows of the fused path are stored this way; FP64
 // rows (zero-count rows, the `post` / cell-table outputs) are always normalised.
-template <bool MODES, int LW, bool NORM>
-__global__ void __launch_bounds__(ROW_WARPS * 32, LW == 32 ? 3 : 2)
+template <bool MODES, bool NORM>
+__global__ void __launch_bounds__(ROW_WARPS * 32, 2)
 lp_rows_fast_kernel(const double *__restrict__ models, int ldm, CellRange cr, const int32_t *__restrict__ row_off,
                     const int32_t *__restrict__ row_cell, const int32_t *__restrict__ row_x,
                     const double4 *__restrict__ rowc, const int32_t *__restrict__ row_snap, CellPrep prep, int K,
                     double sentinel, double *__restrict__ table, int ld_table, int32_t *__restrict__ row_mode, int which,
                     const int32_t *__restrict__ zero_row, const int32_t *__restrict__ based, int write_f64, int zero_compact,
                     int8_t *__restrict__ qtable, int ldq, uint32_t *__restrict__ row_range, int8_t *__restrict__ qbound) {
-    constexpr int RPW = 32 / LW;  // rows per warp
+    constexpr int LW = 16, RPW = 32 / LW;  // lanes per row, rows per warp
     extern __shared__ __align__(16) unsigned char s_dyn[];
     double *s_rows = reinterpret_cast<double *>(s_dyn);                                  // [ROW_WARPS * RPW][KP_TILED]
     uint8_t *s_q = s_dyn + sizeof(double) * ROW_WARPS * RPW * KP_TILED;                  // [ROW_WARPS * RPW][4 * Q_PIECE]
@@ -688,20 +763,7 @@ lp_rows_fast_kernel(const double *__restrict__ models, int ldm, CellRange cr, co
                 *reinterpret_cast<double2 *>(out + k0) = make_double2(v[0], v[1]);
                 *reinterpret_cast<double2 *>(out + k0 + 2) = make_double2(v[2], v[3]);
             }
-            if (qtable && k0 < Q_MAX_K) {
-                uint32_t word[Q_NV], sent;
-                fixed_point_quad(v, word, sent);
-                const int nk = K - k0;  // real grid points in this quad
-                okmask |= (~sent & (nk >= 4 ? 0xFu : nk > 0 ? (1u << nk) - 1u : 0u)) << (4 * jq);
-                // pairs (k0, k0 + 1) and (k0 + 2, k0 + 3) never straddle a piece (Q_PW is even): 16-bit stores
-                uint16_t *dst0 = reinterpret_cast<uint16_t *>(sq + q_offset(k0));
-                uint16_t *dst1 = reinterpret_cast<uint16_t *>(sq + q_offset(k0 + 2));
-#pragma unroll
-                for (int p = 0; p < Q_NV; ++p) {
-                    dst0[(p * Q_PW) >> 1] = (uint16_t)(word[p] & 0xFFFFu);
-                    dst1[(p * Q_PW) >> 1] = (uint16_t)(word[p] >> 16);
-                }
-            }
+            if (qtable && k0 < Q_MAX_K) q_stage_quad<LW>(sq, k0, jq, K, v, okmask);
         }
         if (write_f64 && valid)
             for (int k = kp + l; k < ld_table; k += LW) out[k] = 0.0;
@@ -717,31 +779,42 @@ lp_rows_fast_kernel(const double *__restrict__ models, int ldm, CellRange cr, co
             }
         }
         __syncwarp();
-        if (qtable) {  // the row's planes, 16 bytes per lane and store
-            const uint4 *src = reinterpret_cast<const uint4 *>(sq);
-            uint4 *dst = reinterpret_cast<uint4 *>(qtable + (size_t)row * ldq);
-            if (valid)
-                for (int j = l; j < ldq / 16; j += LW) dst[j] = src[j];
-            // count, first and last of the grid points that are not "log 0" (bit b of a lane <-> k = 4 l + 4 LW (b >> 2) + (b & 3))
-            int n_ok = __popc(okmask), kmin = 0x7fffffff, kmax = -1;
-            if (okmask) {
-                const int b0 = __ffs(okmask) - 1, b1 = 31 - __clz(okmask);
-                kmin = 4 * l + 4 * LW * (b0 >> 2) + (b0 & 3);
-                kmax = 4 * l + 4 * LW * (b1 >> 2) + (b1 & 3);
-            }
-#pragma unroll
-            for (int o = LW / 2; o > 0; o >>= 1) {
-                n_ok += __shfl_xor_sync(0xffffffffu, n_ok, o);
-                kmin = min(kmin, __shfl_xor_sync(0xffffffffu, kmin, o));
-                kmax = max(kmax, __shfl_xor_sync(0xffffffffu, kmax, o));
-            }
-            const uint32_t rr = (n_ok > 0 && kmax - kmin + 1 == n_ok) ? ((uint32_t)kmin | ((uint32_t)kmax << 16)) : Q_RANGE_IRREGULAR;
-            if (l == 0 && valid) row_range[row] = rr;
-            if (qbound && valid) q_bound_row(reinterpret_cast<const int8_t *>(sq), K, rr, qbound + (size_t)row * Q_BW, l, LW);
-        }
+        if (qtable) q_store_row<LW>(sq, okmask, l, K, row, valid, qtable, ldq, row_range, qbound);
         __syncwarp();
         if (MODES && l == 0 && valid) row_mode[row] = (besti == 0x7fffffff) ? 0 : besti;
     }
+}
+
+// ---- fixed-point rows of an FP64 table --------------------------------------------------------------
+// The planes, ranges and bound rows of the rows that lp_rows_kernel and lp_rows_fast_kernel store in FP64 only (local-theta
+// and conc.a2 models, fused_fixed_point = 0), one warp per row.  fixed_point_quad needs no clamp here: its digits are
+// exact for |v| < 1020 and zero for !(v > -1e290) (NaN included), and such a table holds lp(x) in [-752, 0] (v_k / S with
+// 1 <= S <= 2 K, v_k 0 or at least the least denormal), differences of two of them (based_flags_kernel: a based cell's
+// zero-count row has no sentinel), and the sentinel -DBL_MAX / n / 1.1 <= -7e298 (n is an int) less at most 752.
+constexpr int QZ_WARPS = 8;
+__global__ void __launch_bounds__(QZ_WARPS * 32)
+quantize_rows_kernel(const double *__restrict__ table, int ld_table, int K, int64_t n_rows, int8_t *__restrict__ qtable,
+                     int ldq, uint32_t *__restrict__ row_range, int8_t *__restrict__ qbound) {
+    extern __shared__ __align__(16) unsigned char s_dyn[];  // [QZ_WARPS][4 * Q_PIECE]
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int64_t row = (int64_t)blockIdx.x * QZ_WARPS + warp;
+    if (row >= n_rows) return;
+    uint8_t *sq = s_dyn + warp * (4 * Q_PIECE);
+    for (int j = lane; j < (4 * Q_PIECE) / 16; j += 32) reinterpret_cast<uint4 *>(sq)[j] = make_uint4(0u, 0u, 0u, 0u);
+    __syncwarp();
+    const double *src = table + row * ld_table;
+    uint32_t okmask = 0u;
+    for (int k0 = 4 * lane, j = 0; k0 < K; k0 += 4 * 32, ++j) {
+        double v[4];
+        *reinterpret_cast<double2 *>(&v[0]) = *reinterpret_cast<const double2 *>(src + k0);
+        *reinterpret_cast<double2 *>(&v[2]) = *reinterpret_cast<const double2 *>(src + k0 + 2);
+#pragma unroll
+        for (int e = 0; e < 4; ++e)
+            if (k0 + e >= K) v[e] = 0.0;  // beyond the grid: zero digits
+        q_stage_quad<32>(sq, k0, j, K, v, okmask);
+    }
+    __syncwarp();
+    q_store_row<32>(sq, okmask, lane, K, row, true, qtable, ldq, row_range, qbound);
 }
 
 // ---- fixed-point rows of the fused path, cell state in registers -----------------------------------
@@ -1172,6 +1245,15 @@ cudaError_t launch_based_flags(const double *table, int ld_table, int K, double 
     return cudaGetLastError();
 }
 
+cudaError_t launch_quantize_rows(const double *table, int ld_table, int K, int64_t n_rows, int8_t *qtable,
+                                 uint32_t *row_range, int8_t *qbound, cudaStream_t st) {
+    if (n_rows <= 0) return cudaSuccess;
+    if (K > ld_table || ld_table % 4 != 0 || K > Q_MAX_K) return cudaErrorInvalidValue;
+    quantize_rows_kernel<<<(unsigned)((n_rows + QZ_WARPS - 1) / QZ_WARPS), QZ_WARPS * 32, QZ_WARPS * 4 * Q_PIECE, st>>>(
+        table, ld_table, K, n_rows, qtable, q_row_bytes(K), row_range, qbound);
+    return cudaGetLastError();
+}
+
 namespace {
 
 // The row kernels of the table take their rows' bounds on the device: the grid is sized for the cells (hundreds of rows
@@ -1195,8 +1277,8 @@ cudaError_t launch_row_kernel(const RowArgs &a, CellRange cr, int which, int32_t
         };
         // rows that exist in fixed point only need no normalising constant
         if (row_mode)
-            return write_f64 ? launch(lp_rows_fast_kernel<true, 16, true>) : launch(lp_rows_fast_kernel<true, 16, false>);
-        return write_f64 ? launch(lp_rows_fast_kernel<false, 16, true>) : launch(lp_rows_fast_kernel<false, 16, false>);
+            return write_f64 ? launch(lp_rows_fast_kernel<true, true>) : launch(lp_rows_fast_kernel<true, false>);
+        return write_f64 ? launch(lp_rows_fast_kernel<false, true>) : launch(lp_rows_fast_kernel<false, false>);
     }
     size_t smem = (size_t)ROW_WARPS * a.K * sizeof(double);
     if (smem > 48 * 1024) {

@@ -287,8 +287,8 @@ def classified(gi, local=False):
 # ---- CPU ----------------------------------------------------------------------------------------------------------------
 def test_decoder_round_trip():
     """the numpy packing and decoder are inverse: X = rint(v 2^29) for |v| <= 752 (ties to even, as the addition of the
-    magic constant rounds), the "log 0" element is five zero digits, and the digits are those quantize_rows_kernel
-    writes"""
+    magic constant rounds), the "log 0" element is five zero digits, and the digits are the balanced radix-256 digits
+    of a plain digit loop up to the extremes of five digits"""
     rng = np.random.default_rng(1)
     for K in (1, 16, 101, 102, 103, 401, 408):
         v = rng.uniform(-752.0, 752.0, size=(7, K))
@@ -307,7 +307,7 @@ def test_decoder_round_trip():
         used = np.zeros(q_row_bytes(K), bool)
         used[(_plane_index(K)[:, None] + Q_PW * np.arange(Q_NV)[None, :]).ravel()] = True
         assert np.all(q[:, ~used] == 0)
-    # the digits of quantize_rows_kernel: d = (int8)(x & 0xFF), x = (x - d) >> 8
+    # the digit loop: d = (int8)(x & 0xFF), x = (x - d) >> 8
     x = np.array([0, 1, -1, 127, 128, -128, -129, 752 * 2 ** 29, -752 * 2 ** 29,
                   0x7F7F7F7F7F, -0x8080808080], np.int64)  # the last two: the extremes of five digits
     q = np.zeros((len(x), q_row_bytes(1)), np.int8)
