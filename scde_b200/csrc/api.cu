@@ -2002,15 +2002,21 @@ struct scde_b200_diff_job {
     int64_t known_rows = 0;          // table rows of the last completed run of this job (0: unknown): the next run needs no
                                      // size read-back -- same counts, same rows
     bool rows_unchecked = false;     // the last run used known_rows as the capacity; download verifies it
-    int copy_chunks = 0;             // chunked H2D of the counts in flight on the context's copy stream:
-    std::vector<int> copy_bounds;    // chunk i holds the cells [copy_bounds[i], copy_bounds[i + 1])
-    int split_chunks = 0;            // > 0: the chunks [0, split_chunks) hold every cell of the first group, whose joint
-                                     // runs before the rest of the front (so it hides the second half of the upload)
-    int64_t front_cap = 0;           // row capacity chosen by the chunked front
     const int32_t *boot_ptr[4] = {nullptr, nullptr, nullptr, nullptr};  // draws as the device reads them
     std::vector<int32_t> ids[2];                 // cells of the two groups
     std::unique_ptr<int32_t[]> gen[4];           // generated draws (resident job), alive until their uploads have completed
-    const scde_b200_diff_args *deferred_args = nullptr;  // one-shot call: the draws are still to be generated and uploaded
+};
+
+// A job owned by a scope: released as scde_b200_diff_free releases it, on every return
+struct JobFree {
+    void operator()(scde_b200_diff_job *j) const { scde_b200_diff_free(j->owner, j); }
+};
+using JobPtr = std::unique_ptr<scde_b200_diff_job, JobFree>;
+
+// Host wall-clock of the trace lines on stderr (scde_b200_options.trace): milliseconds since construction
+struct WallClock {
+    const std::chrono::steady_clock::time_point t0 = std::chrono::steady_clock::now();
+    double ms() const { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count(); }
 };
 
 // Bootstrap draws of the group joints (local indices) and, with a batch factor, of the composition-sampled joints (global
@@ -2095,88 +2101,103 @@ int upload_draws(scde_b200_ctx *ctx, scde_b200_diff_job *j, const scde_b200_diff
     return SCDE_B200_OK;
 }
 
-constexpr int N_COUNT_CHUNKS_DEFAULT = 8;
-static int n_count_chunks(const scde_b200_ctx *ctx) {
-    const int n = ctx->opt.count_chunks > 0 ? ctx->opt.count_chunks : N_COUNT_CHUNKS_DEFAULT;
-    return n < 1 ? 1 : (n > 64 ? 64 : n);
-}
-
-// Queue the H2D of the shard's count matrix on the copy stream in N_COUNT_CHUNKS cell ranges, one event per range, so
-// the 22 ms of PCIe time at config 4 run under the front kernels.
-int start_count_copies(scde_b200_ctx *ctx, scde_b200_diff_job *j, const int32_t *counts_host, int64_t ld_host) {
-    const int G = j->G, C = j->C;
-    const int N_COUNT_CHUNKS = n_count_chunks(ctx);
-    if (!ctx->copy_stream) SCDE_CUDA(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
-    while ((int)ctx->copy_events.size() < N_COUNT_CHUNKS + 1) {
-        cudaEvent_t e;
-        SCDE_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        ctx->copy_events.push_back(e);
-    }
-    // the copy stream may overwrite the counts buffer only after earlier work on the compute stream is done with it
-    SCDE_CUDA(cudaEventRecord(ctx->copy_events[N_COUNT_CHUNKS], ctx->stream));
-    SCDE_CUDA(cudaStreamWaitEvent(ctx->copy_stream, ctx->copy_events[N_COUNT_CHUNKS], 0));
-    // Chunk sizes: the front ends at max(last copy + the last chunk's kernels, first chunk's arrival + all kernels), so
-    // the first and the last chunk are small (1/20 and 1/16 of the cells) and the ones between share the rest.
-    // Split front: when every cell of the first group lies in the leading part of the matrix (the usual layout: cells
-    // ordered by group), a chunk boundary is put right behind that group's last cell.  The first group's joint then
-    // runs as soon as those chunks are processed -- under the upload of the rest, which is what bounds the call when
-    // several ranks share the host's PCIe bandwidth (eight ranks: 35-50 ms for the 1.2 GB instead of 22).
-    std::vector<int> &bounds = j->copy_bounds;
-    bounds.assign(1, 0);
-    j->split_chunks = 0;
-    auto add_equal = [&](int lo, int hi, int n) {  // n chunks over [lo, hi), boundaries on multiples of 32, hi included
-        n = n < 1 ? 1 : n;
-        const int step = round_up((hi - lo + n - 1) / n, 32);
+// The cell chunks of the one-shot call's count upload: n of them (1..64) over C cells, chunk i holding the cells
+// [bounds[i], bounds[i + 1]).  Chunk sizes: the front ends at max(last copy + the last chunk's kernels, first chunk's
+// arrival + all kernels), so the first and the last chunk are small (1/20 and 1/16 of the cells) and the ones between
+// share the rest (uniform: equal chunks).
+// Split front: when every cell of the first group (last0: its last cell; -1: no split) lies in the leading part of the
+// matrix (the usual layout: cells ordered by group), a chunk boundary is put right behind that group's last cell and
+// *split counts the chunks before it (0: no split).  The first group's joint then runs as soon as those chunks are
+// processed -- under the upload of the rest, which is what bounds the call when several ranks share the host's PCIe
+// bandwidth (eight ranks: 35-50 ms for the 1.2 GB instead of 22).
+static std::vector<int> count_chunk_bounds(int C, int n, int last0, bool uniform, int *split) {
+    std::vector<int> bounds(1, 0);
+    *split = 0;
+    auto add_equal = [&](int lo, int hi, int m) {  // m chunks over [lo, hi), boundaries on multiples of 32, hi included
+        m = m < 1 ? 1 : m;
+        const int step = round_up((hi - lo + m - 1) / m, 32);
         for (int c = lo + step; c < hi; c += step) bounds.push_back(c);
         bounds.push_back(hi);
     };
-    int split = 0;
-    if (!j->ids[0].empty() && ctx->opt.split_front) {
-        int last0 = 0;
-        for (int c : j->ids[0]) last0 = c > last0 ? c : last0;
-        split = round_up(last0 + 1, 32);
-    }
-    if (N_COUNT_CHUNKS >= 4 && C >= 64 * N_COUNT_CHUNKS && !ctx->opt.uniform_chunks) {
+    const int split_cell = last0 >= 0 ? round_up(last0 + 1, 32) : 0;
+    if (n >= 4 && C >= 64 * n && !uniform) {
         const int first = round_up(C / 20, 32), last = round_up(C / 16, 32);
-        if (split >= 2 * first && split <= C - 2 * last && split <= (C / 4) * 3) {
-            int nA = (int)((double)N_COUNT_CHUNKS * split / C + 0.5);
-            nA = nA < 2 ? 2 : (nA > N_COUNT_CHUNKS - 2 ? N_COUNT_CHUNKS - 2 : nA);
+        if (split_cell >= 2 * first && split_cell <= C - 2 * last && split_cell <= (C / 4) * 3) {
+            int nA = (int)((double)n * split_cell / C + 0.5);
+            nA = nA < 2 ? 2 : (nA > n - 2 ? n - 2 : nA);
             bounds.push_back(first);
-            add_equal(first, split, nA - 1);
-            j->split_chunks = (int)bounds.size() - 1;
-            add_equal(split, C - last - ((C - last) % 32), N_COUNT_CHUNKS - nA - 1);
+            add_equal(first, split_cell, nA - 1);
+            *split = (int)bounds.size() - 1;
+            add_equal(split_cell, C - last - ((C - last) % 32), n - nA - 1);
             bounds.push_back(C);
         } else {
-            const int mid = round_up((C - first - last + N_COUNT_CHUNKS - 3) / (N_COUNT_CHUNKS - 2), 32);
+            const int mid = round_up((C - first - last + n - 3) / (n - 2), 32);
             bounds.push_back(first);
-            for (int i = 0; i < N_COUNT_CHUNKS - 2 && bounds.back() + mid < C - last; ++i) bounds.push_back(bounds.back() + mid);
+            for (int i = 0; i < n - 2 && bounds.back() + mid < C - last; ++i) bounds.push_back(bounds.back() + mid);
             if (bounds.back() < C - last) bounds.push_back(C - last - ((C - last) % 32));
             if (bounds.back() <= bounds[bounds.size() - 2]) bounds.pop_back();
             bounds.push_back(C);
         }
     } else {
-        const int chunk = round_up((C + N_COUNT_CHUNKS - 1) / N_COUNT_CHUNKS, 32);
+        const int chunk = round_up((C + n - 1) / n, 32);
         for (int c0 = chunk; c0 < C; c0 += chunk) bounds.push_back(c0);
         bounds.push_back(C);
     }
-    while ((int)ctx->copy_events.size() < (int)bounds.size() + 1) {
-        cudaEvent_t e;
-        SCDE_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        ctx->copy_events.push_back(e);
-    }
-    j->copy_chunks = 0;
-    for (int n_ch = 0; n_ch + 1 < (int)bounds.size(); ++n_ch) {
-        const int c0 = bounds[n_ch], n = bounds[n_ch + 1] - c0;
-        // counted before it is queued: if a later call fails, the caller (fail() of diff_upload_impl) drains the copy stream
-        // whenever copy_chunks != 0 -- the copy engine must not read the caller's buffer after the call has returned
-        j->copy_chunks = n_ch + 1;
-        SCDE_CUDA(cudaMemcpy2DAsync(j->ws->counts.p + (size_t)c0 * G, sizeof(int32_t) * G, counts_host + (size_t)c0 * ld_host,
-                                    sizeof(int32_t) * (size_t)ld_host, sizeof(int32_t) * G, n, cudaMemcpyHostToDevice,
-                                    ctx->copy_stream));
-        SCDE_CUDA(cudaEventRecord(ctx->copy_events[n_ch], ctx->copy_stream));
-    }
-    return SCDE_B200_OK;
+    return bounds;
 }
+
+// The one-shot call's H2D of its count matrix, in cell chunks on the context's copy stream with one event per chunk, so
+// the 22 ms of PCIe time at config 4 run under the front kernels.  It lives for the length of the call: the call must not
+// return while the copy engine may still read the caller's buffer, so whatever it has queued is drained on destruction.
+struct CountUpload {
+    scde_b200_ctx *ctx;
+    std::vector<int> bounds;  // chunk i holds the cells [bounds[i], bounds[i + 1])
+    int split = 0;            // > 0: the chunks [0, split) hold every cell of the first group
+    int queued = 0;           // copies queued on the copy stream
+
+    explicit CountUpload(scde_b200_ctx *c) : ctx(c) {}
+    CountUpload(const CountUpload &) = delete;
+    CountUpload &operator=(const CountUpload &) = delete;
+    ~CountUpload() { drain(); }
+
+    int chunks() const { return (int)bounds.size() - 1; }
+
+    // the job's counts (G x C, rows [g0, g1) of the caller's matrix at counts_host, leading dimension ld_host)
+    int start(const scde_b200_diff_job &j, const int32_t *counts_host, int64_t ld_host) {
+        const int G = j.G, C = j.C;
+        const int n = ctx->opt.count_chunks > 0 ? ctx->opt.count_chunks : default_options().count_chunks;
+        bounds = count_chunk_bounds(C, n, ctx->opt.split_front ? j.ids[0].back() : -1, ctx->opt.uniform_chunks != 0,
+                                    &split);
+        SCDE_CUDA(j.ws->counts.ensure((size_t)G * C));
+        if (!ctx->copy_stream) SCDE_CUDA(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
+        while ((int)ctx->copy_events.size() < chunks() + 1) {
+            cudaEvent_t e;
+            SCDE_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+            ctx->copy_events.push_back(e);
+        }
+        // the copy stream may overwrite the counts buffer only after earlier work on the compute stream is done with it
+        SCDE_CUDA(cudaEventRecord(ctx->copy_events[chunks()], ctx->stream));
+        SCDE_CUDA(cudaStreamWaitEvent(ctx->copy_stream, ctx->copy_events[chunks()], 0));
+        for (int i = 0; i < chunks(); ++i) {
+            const int c0 = bounds[i], m = bounds[i + 1] - c0;
+            ++queued;  // counted before it is queued: a failed call still drains
+            SCDE_CUDA(cudaMemcpy2DAsync(j.ws->counts.p + (size_t)c0 * G, sizeof(int32_t) * G,
+                                        counts_host + (size_t)c0 * ld_host, sizeof(int32_t) * (size_t)ld_host,
+                                        sizeof(int32_t) * G, m, cudaMemcpyHostToDevice, ctx->copy_stream));
+            SCDE_CUDA(cudaEventRecord(ctx->copy_events[i], ctx->copy_stream));
+        }
+        return SCDE_B200_OK;
+    }
+
+    // the compute stream waits for the chunks [lo, hi)
+    int wait(int lo, int hi) const {
+        for (int i = lo; i < hi; ++i) SCDE_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->copy_events[i], 0));
+        return SCDE_B200_OK;
+    }
+
+    // the host waits until every queued copy has landed
+    cudaError_t drain() const { return queued ? cudaStreamSynchronize(ctx->copy_stream) : cudaSuccess; }
+};
 
 // the genes [g0, g1) a call processes: [gene_begin, gene_end), all of them when both are 0
 static int gene_range(const scde_b200_diff_args *a, int *g0, int *g1) {
@@ -2190,11 +2211,10 @@ static int gene_range(const scde_b200_diff_args *a, int *g0, int *g1) {
     return SCDE_B200_OK;
 }
 
-// defer_counts: the count matrix is not copied here (the one-shot call overlaps its upload with the table build)
-static int diff_upload_impl(scde_b200_ctx *ctx, const scde_b200_diff_args *a, int32_t want_posteriors,
-                            scde_b200_diff_job **out, bool defer_counts) {
-    if (!a || !out) return SCDE_B200_EINVAL;
-    *out = nullptr;
+// A job with everything on the device but its count matrix and its draws, which the caller uploads: the resident job in
+// one copy, the one-shot call in chunks overlapped with the table build
+static int diff_upload_impl(scde_b200_ctx *ctx, const scde_b200_diff_args *a, int32_t want_posteriors, JobPtr &out) {
+    if (!a) return SCDE_B200_EINVAL;
     if (!a->counts || !a->models || !a->prior_x || !a->prior_y || !a->group || a->n_genes < 1 || a->n_cells < 1 ||
         a->n_grid < 2 || a->n_boot < 1) {
         set_error("expression_difference: bad arguments");
@@ -2223,25 +2243,9 @@ static int diff_upload_impl(scde_b200_ctx *ctx, const scde_b200_diff_args *a, in
     }
     cudaStream_t st = ctx->stream;
     TRY(acquire_workspace(ctx));
-    scde_b200_diff_job *j = new scde_b200_diff_job();
+    JobPtr j(new scde_b200_diff_job());
     j->ws = ctx->ws;
     j->owner = ctx;
-    auto fail = [&](int r) {
-        if (j->copy_chunks) cudaStreamSynchronize(ctx->copy_stream);  // the copy engine reads the caller's buffer
-        ctx->ws_busy = false;
-        delete j;
-        return r;
-    };
-#define JTRY(x)                                \
-    do {                                       \
-        int _r = (x);                          \
-        if (_r != SCDE_B200_OK) return fail(_r); \
-    } while (0)
-#define JCUDA(x)                                                                    \
-    do {                                                                            \
-        cudaError_t _e = (x);                                                       \
-        if (_e != cudaSuccess) return fail(cuda_fail(_e, #x, __FILE__, __LINE__));   \
-    } while (0)
     j->G = G;
     j->C = C;
     j->K = K;
@@ -2250,205 +2254,159 @@ static int diff_upload_impl(scde_b200_ctx *ctx, const scde_b200_diff_args *a, in
     j->has_batch = has_batch;
     j->n_levels = has_batch ? a->n_batch_levels : 0;
     j->n_zero = a->n_zero;
-    // counts shard: rows [g0, g1) of every column
-    const bool trace = ctx->opt.trace != 0;
-    const auto tu0 = std::chrono::steady_clock::now();
-    JCUDA(j->ws->counts.ensure((size_t)G * C));
-    const auto tu1 = std::chrono::steady_clock::now();
-    if (!defer_counts)
-        JCUDA(cudaMemcpy2DAsync(j->ws->counts.p, sizeof(int32_t) * G, a->counts + g0, sizeof(int32_t) * (size_t)a->n_genes,
-                                sizeof(int32_t) * G, C, cudaMemcpyHostToDevice, st));
-    if (trace && !defer_counts) {
-        JCUDA(cudaStreamSynchronize(st));
-        const auto tu2 = std::chrono::steady_clock::now();
-        fprintf(stderr, "[scde_b200] upload: counts buffer %.2f ms, counts H2D (%.1f MB) %.2f ms\n",
-                std::chrono::duration<double, std::milli>(tu1 - tu0).count(), sizeof(int32_t) * (double)G * C / 1e6,
-                std::chrono::duration<double, std::milli>(tu2 - tu1).count());
-    }
-    JTRY(upload_models(j->models, a->models, C, a->local_theta, a->square_logit_conc, st));
+    TRY(upload_models(j->models, a->models, C, a->local_theta, a->square_logit_conc, st));
     if (has_batch && a->batch_models && a->batch_models != a->models)
-        JTRY(upload_models(j->bmodels, a->batch_models, C, a->batch_local_theta, a->batch_square_logit_conc, st));
-    JTRY(upload(j->prior_y, a->prior_y, (size_t)K, st));
+        TRY(upload_models(j->bmodels, a->batch_models, C, a->batch_local_theta, a->batch_square_logit_conc, st));
+    TRY(upload(j->prior_y, a->prior_y, (size_t)K, st));
     const std::vector<double> mag = grid_magnitudes(a->prior_x, K);
-    JTRY(upload(j->mag, mag.data(), (size_t)K, st));
+    TRY(upload(j->mag, mag.data(), (size_t)K, st));
     for (int i = 0; i < 2; ++i) {
         j->n_group[i] = (int)ids[i].size();
-        JTRY(upload(j->cell_ids[i], ids[i].data(), ids[i].size(), st));
+        TRY(upload(j->cell_ids[i], ids[i].data(), ids[i].size(), st));
     }
-    // draws: generated (host RNG, 1.3 ms per group at config 4) and uploaded now, or -- one-shot call -- while the front
-    // kernels run (upload_draws is then called by diff_run_impl)
     j->ids[0] = ids[0];
     j->ids[1] = ids[1];
     j->chunks = draw_chunks_of(a->n_genes, a->draw_chunks, a->seed, g0, g1);
-    if (j->chunks.n_sets() > 1) JTRY(upload(j->gene_set, j->chunks.gene_set.data(), j->chunks.gene_set.size(), st));
-    if (defer_counts)
-        j->deferred_args = a;
-    else
-        JTRY(upload_draws(ctx, j, a));
+    if (j->chunks.n_sets() > 1) TRY(upload(j->gene_set, j->chunks.gene_set.data(), j->chunks.gene_set.size(), st));
     {
         const std::vector<int32_t> zi = zero_slice(a->zero_index, a->n_zero, g0, G);
-        JTRY(validate_index(zi.data(), zi.size(), 1, 2 * K, "zero_index"));
-        JTRY(upload(j->zi, zi.data(), zi.size(), st));
+        TRY(validate_index(zi.data(), zi.size(), 1, 2 * K, "zero_index"));
+        TRY(upload(j->zi, zi.data(), zi.size(), st));
         if (has_batch) {
             const std::vector<int32_t> za = zero_slice(a->zero_index_adjusted, a->n_zero, g0, G);
-            JTRY(validate_index(za.data(), za.size(), 1, 4 * K - 2, "zero_index_adjusted"));
-            JTRY(upload(j->zi_adj, za.data(), za.size(), st));
+            TRY(validate_index(za.data(), za.size(), 1, 4 * K - 2, "zero_index_adjusted"));
+            TRY(upload(j->zi_adj, za.data(), za.size(), st));
         }
-        JCUDA(cudaStreamSynchronize(st));
+        SCDE_CUDA(cudaStreamSynchronize(st));
     }
     const int ld = table_ld(K), nout = 2 * K - 1, ldo = round_up(nout, 8), nadj = 2 * nout - 1, lda = round_up(nadj, 8);
-    for (int i = 0; i < (has_batch ? 4 : 2); ++i) JCUDA(j->ws->jp[i].ensure((size_t)G * ld));
-    JCUDA(j->idx.ensure((size_t)3 * G));
-    JCUDA(j->z.ensure((size_t)G));
-    JCUDA(j->status.ensure(3));
-    if (want_posteriors || has_batch) JCUDA(j->ws->post.ensure((size_t)G * ldo));
+    for (int i = 0; i < (has_batch ? 4 : 2); ++i) SCDE_CUDA(j->ws->jp[i].ensure((size_t)G * ld));
+    SCDE_CUDA(j->idx.ensure((size_t)3 * G));
+    SCDE_CUDA(j->z.ensure((size_t)G));
+    SCDE_CUDA(j->status.ensure(3));
+    if (want_posteriors || has_batch) SCDE_CUDA(j->ws->post.ensure((size_t)G * ldo));
     if (has_batch) {
-        JCUDA(j->ws->bpost.ensure((size_t)G * ldo));
-        JCUDA(j->bidx.ensure((size_t)3 * G));
-        JCUDA(j->bz.ensure((size_t)G));
-        JCUDA(j->aidx.ensure((size_t)3 * G));
-        JCUDA(j->az.ensure((size_t)G));
-        if (want_posteriors) JCUDA(j->ws->apost.ensure((size_t)G * lda));
+        SCDE_CUDA(j->ws->bpost.ensure((size_t)G * ldo));
+        SCDE_CUDA(j->bidx.ensure((size_t)3 * G));
+        SCDE_CUDA(j->bz.ensure((size_t)G));
+        SCDE_CUDA(j->aidx.ensure((size_t)3 * G));
+        SCDE_CUDA(j->az.ensure((size_t)G));
+        if (want_posteriors) SCDE_CUDA(j->ws->apost.ensure((size_t)G * lda));
     }
-    JCUDA(cudaStreamSynchronize(st));
-    // last: the small uploads above share the one H2D copy engine with these 1.2 GB and would queue behind them
-    if (defer_counts) JTRY(start_count_copies(ctx, j, a->counts + g0, a->n_genes));
-    *out = j;
+    SCDE_CUDA(cudaStreamSynchronize(st));
+    out = std::move(j);
     return SCDE_B200_OK;
-#undef JTRY
-#undef JCUDA
 }
 
-// Chunked front of the one-shot call: the count matrix goes up in N_CHUNKS cell ranges on the copy stream, and every
-// range is deduplicated and its table rows are built on the compute stream as soon as it has landed, so the 1.2 GB H2D of
-// config 4 (22 ms at PCIe rate) hides behind the row kernels.  Row offsets are chunk-local scans carried forward on the
-// device; the row-level kernels read their bounds there (CellRange), so nothing waits for the host except one 4-byte read
-// after the first chunk: its row count sizes the buffers (x 1.25).  If the estimate turns out too small the kernels stop
-// at the capacity and *done stays false: the caller rebuilds index and table the classic way from the resident counts.
-// phase 0: the chunks [0, split_chunks) -- all of them without a split; phase 1: the rest (split front only).  A phase
-// returns with the compute stream idle and its rows checked against the capacity, so the caller may queue a joint on them.
-static int front_chunked(scde_b200_ctx *ctx, scde_b200_diff_job *j, ContractChoice k, int phase, bool *done) {
-    *done = false;
+// the joint of group i: cells of one factor level, draws are local indices (R/functions.R:372-374)
+static int group_joint(scde_b200_ctx *ctx, scde_b200_diff_job *j, ContractChoice k, int i) {
+    const Joint jt{j->boot_ptr[i], j->D[i], j->ws->jp[i].p};
+    return run_joint(ctx, k, j->ws->table, j->cell_ids[i].p, j->n_group[i], &jt, 1, j->n_boot,
+                     DrawSets{j->chunks.n_sets(), j->gene_set.p}, (double)j->n_boot, table_ld(j->K), j->ws->scr,
+                     j->status.p + i, &j->timer, true);
+}
+
+// What the front of the one-shot call has done of its run
+struct FrontDone {
+    bool table = false;   // the index and the table of every cell
+    bool joint0 = false;  // the first group's joint (split front)
+};
+
+// Chunked front of the one-shot call: as soon as a chunk of the count matrix has landed (CountUpload), the compute stream
+// deduplicates it and builds its table rows, so the 1.2 GB H2D of config 4 (22 ms at PCIe rate) hides behind the row
+// kernels.  Row offsets are chunk-local scans carried forward on the device; the row-level kernels read their bounds there
+// (CellRange), so nothing waits for the host except one 4-byte read after the first chunk: its row count sizes the buffers
+// (x 1.25).  Only the compact table is built chunk by chunk: its rows need no pass after the last chunk, and a row
+// capacity estimated too large costs fixed-point rows only; any other table is built by diff_run_impl once the whole
+// matrix has landed.
+// Split front: the chunks [0, up.split) are processed first and their rows checked against the capacity; the first group's
+// joint then runs while the rest of the matrix is still arriving.  The draws of a are generated while the first chunks'
+// kernels run, into the mapped pinned staging when the front is split.  If the estimate turns out too small the kernels
+// stop at the capacity and *done says what is left: diff_run_impl rebuilds index and table the classic way from the
+// resident counts, and repeats the first joint on the new row ids.
+static int front_chunked(scde_b200_ctx *ctx, scde_b200_diff_job *j, ContractChoice k, CountUpload &up,
+                         const scde_b200_diff_args *a, FrontDone *done) {
     LpTable &t = j->ws->table;
-    const int G = j->G, C = j->C;
+    const int G = j->G, C = j->C, n_ch = up.chunks();
     cudaStream_t st = ctx->stream;
     StageTimer &tm = j->timer;
     const TableRequest req = diff_table(j->models, j->mag.p, j->K, k);
-    // the copies are already in flight (start_count_copies); every path below waits for them on the compute stream.  Only
-    // the compact table is built chunk by chunk: its rows need no pass after the last chunk, and a row capacity estimated
-    // too large costs fixed-point rows only.
-    const bool pipelined = plan_table(ctx, req).compact() && C >= 64 * j->copy_chunks && ctx->opt.pipeline_front;
-    if (!pipelined) {
-        j->split_chunks = 0;
-        for (int i = 0; i < j->copy_chunks; ++i) SCDE_CUDA(cudaStreamWaitEvent(st, ctx->copy_events[i], 0));
-        return SCDE_B200_OK;
+    if (!(plan_table(ctx, req).compact() && C >= 64 * n_ch && ctx->opt.pipeline_front)) {
+        TRY(up.wait(0, n_ch));
+        return upload_draws(ctx, j, a);
     }
-    const bool split = j->split_chunks > 0 && j->split_chunks < j->copy_chunks;
-    const int ch_lo = phase == 0 ? 0 : j->split_chunks, ch_hi = (phase == 0 && split) ? j->split_chunks : j->copy_chunks;
-    const bool last_phase = ch_hi == j->copy_chunks;
-    auto drain = [&](int r) {  // never return while the copy engine may still read the caller's buffer
-        cudaStreamSynchronize(ctx->copy_stream);
-        return r;
-    };
-#define FTRY(x)                                   \
-    do {                                          \
-        int _r = (x);                             \
-        if (_r != SCDE_B200_OK) return drain(_r); \
-    } while (0)
-#define FCUDA(x)                                                                    \
-    do {                                                                            \
-        cudaError_t _e = (x);                                                       \
-        if (_e != cudaSuccess) return drain(cuda_fail(_e, #x, __FILE__, __LINE__));  \
-    } while (0)
-    const bool trace = ctx->opt.trace != 0;
-    const auto tf0 = std::chrono::steady_clock::now();
-    auto since = [&] { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - tf0).count(); };
-    double tr_first = 0, tr_queued = 0, tr_draws = 0, tr_front = 0, tr_copy = 0;
-    int e0 = 0;
-    if (phase == 0) {
-        FTRY(index_buffers(ctx, t, G, C));
-        FTRY(begin_table(ctx, t, req, &tm));
-        j->front_cap = 0;
-    }
-    int64_t cap = j->front_cap;
-    // phase 1 follows the first group's joint (29 ms at config 4), by which time the rest of the matrix has landed: its
-    // chunks are processed as one range (full grids, a sixth of the launches)
-    const int ch_step = phase == 1 ? ch_hi - ch_lo : 1;
-    for (int i = ch_lo; i < ch_hi; i += ch_step) {
-        const int c0 = j->copy_bounds[i], n = j->copy_bounds[i + ch_step] - c0;
-        const int32_t *cnt = j->ws->counts.p + (size_t)c0 * G;
-        for (int e = i; e < i + ch_step; ++e) FCUDA(cudaStreamWaitEvent(st, ctx->copy_events[e], 0));
-        e0 = tm.begin(st);
-        uint32_t *bits = t.dedup_bits.p + dedup_scratch_words(c0) * (c0 > 0);
-        FCUDA(launch_dedup_count(cnt, G, 0, G, n, t.n_unique.p + c0, t.err.p, bits, st));
-        FCUDA(launch_exclusive_scan(t.n_unique.p + c0, t.row_off.p + c0, n, i ? t.row_off.p + c0 : nullptr, st));
-        if (i == 0) {
-            int32_t rows0 = 0;
-            FCUDA(cudaMemcpyAsync(&rows0, t.row_off.p + n, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-            FCUDA(cudaStreamSynchronize(st));
-            tr_first = since();
-            cap = (int64_t)((double)rows0 * C / n * 1.25) + 4096;
-            const int64_t have = (int64_t)(t.q.cap / (size_t)q_row_bytes(t.K));  // a workspace from an earlier call
-            if (have > cap) cap = have;
-            if (cap > 0x7fffffff) cap = 0x7fffffff;
-            FTRY(reserve_rows(t, (size_t)cap));
-            FCUDA(t.row_x.ensure((size_t)cap));
-            j->front_cap = cap;
+    const bool split = up.split > 0;
+    TRY(index_buffers(ctx, t, G, C));
+    TRY(begin_table(ctx, t, req, &tm));
+    int64_t cap = 0;
+    for (int part = 0; part < (split ? 2 : 1); ++part) {
+        // the rest of a split front follows the first group's joint (29 ms at config 4), by which time it has landed: its
+        // chunks are processed as one range (full grids, a sixth of the launches)
+        const int lo = part ? up.split : 0, hi = split && !part ? up.split : n_ch, step = part ? hi - lo : 1;
+        const WallClock clk;
+        double tr_first = 0, tr_copy = 0;
+        for (int i = lo; i < hi; i += step) {
+            const int c0 = up.bounds[i], n = up.bounds[i + step] - c0;
+            const int32_t *cnt = j->ws->counts.p + (size_t)c0 * G;
+            TRY(up.wait(i, i + step));
+            const int e0 = tm.begin(st);
+            uint32_t *bits = t.dedup_bits.p + dedup_scratch_words(c0) * (c0 > 0);
+            SCDE_CUDA(launch_dedup_count(cnt, G, 0, G, n, t.n_unique.p + c0, t.err.p, bits, st));
+            SCDE_CUDA(launch_exclusive_scan(t.n_unique.p + c0, t.row_off.p + c0, n, i ? t.row_off.p + c0 : nullptr, st));
+            if (i == 0) {
+                int32_t rows0 = 0;
+                SCDE_CUDA(cudaMemcpyAsync(&rows0, t.row_off.p + n, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+                SCDE_CUDA(cudaStreamSynchronize(st));
+                tr_first = clk.ms();
+                cap = (int64_t)((double)rows0 * C / n * 1.25) + 4096;
+                const int64_t have = (int64_t)(t.q.cap / (size_t)q_row_bytes(t.K));  // a workspace from an earlier call
+                if (have > cap) cap = have;
+                if (cap > 0x7fffffff) cap = 0x7fffffff;
+                TRY(reserve_rows(t, (size_t)cap));
+                SCDE_CUDA(t.row_x.ensure((size_t)cap));
+            }
+            SCDE_CUDA(launch_dedup_emit(cnt, G, 0, G, n, t.row_off.p + c0, t.row_x.p, t.ridx.p + c0, t.ld_ridx, t.err.p, cap,
+                                        bits, st));
+            tm.end(SCDE_B200_T_DEDUP, e0, st, 5);
+            TRY(table_rows(ctx, t, j->models, CellRange{c0, c0 + n, cap}, &tm));
         }
-        FCUDA(launch_dedup_emit(cnt, G, 0, G, n, t.row_off.p + c0, t.row_x.p, t.ridx.p + c0, t.ld_ridx, t.err.p, cap, bits,
-                                st));
-        tm.end(SCDE_B200_T_DEDUP, e0, st, 5);
-        FTRY(table_rows(ctx, t, j->models, CellRange{c0, c0 + n, cap}, &tm));
+        const double tr_queued = clk.ms();
+        if (ctx->opt.trace && hi == n_ch) {
+            SCDE_CUDA(up.drain());
+            tr_copy = clk.ms();
+        }
+        if (part == 0) TRY(upload_draws(ctx, j, a, split));  // host RNG work while the kernels queued above run
+        const double tr_draws = clk.ms();
+        int32_t total = 0, err = 0;
+        SCDE_CUDA(cudaMemcpyAsync(&total, t.row_off.p + up.bounds[hi], sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+        SCDE_CUDA(cudaMemcpyAsync(&err, t.err.p, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+        SCDE_CUDA(cudaStreamSynchronize(st));
+        if (ctx->opt.trace)
+            fprintf(stderr, "[scde_b200] front%s: first chunk counted %.2f ms, chunks queued %.2f, copies done %.2f, draws staged (incl. wait) %.2f, done %.2f\n",
+                    !split ? "" : (part == 0 ? " (first group's chunks)" : " (rest)"), tr_first, tr_queued, tr_copy, tr_draws,
+                    clk.ms());
+        TRY(dedup_error(err));
+        if (total < 0 || (int64_t)total > cap) {  // more rows than estimated
+            if (done->joint0) {  // its row ids change with the rebuilt table
+                done->joint0 = false;
+                SCDE_CUDA(cudaMemsetAsync(j->ws->scr.total.p, 0, 5 * sizeof(unsigned long long), st));
+            }
+            return up.wait(hi, n_ch);  // the rebuild reads every count
+        }
+        t.n_rows = total;
+        if (split && part == 0) {  // every row of the first group's cells is built and within the capacity
+            TRY(group_joint(ctx, j, k, 0));
+            done->joint0 = true;
+        }
     }
-    tr_queued = since();
-    if (trace && last_phase) {
-        cudaStreamSynchronize(ctx->copy_stream);
-        tr_copy = since();
-    }
-    if (j->deferred_args) {  // the bootstrap draws: host RNG work while the kernels queued above run
-        const scde_b200_diff_args *da = j->deferred_args;
-        j->deferred_args = nullptr;
-        FTRY(upload_draws(ctx, j, da, split));
-    }
-    tr_draws = since();
-    int32_t total = 0, err = 0;
-    FCUDA(cudaMemcpyAsync(&total, t.row_off.p + j->copy_bounds[ch_hi], sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    FCUDA(cudaMemcpyAsync(&err, t.err.p, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    FCUDA(cudaStreamSynchronize(st));
-    if (last_phase) FCUDA(cudaStreamSynchronize(ctx->copy_stream));
-    tr_front = since();
-    if (trace)
-        fprintf(stderr, "[scde_b200] front%s: first chunk counted %.2f ms, chunks queued %.2f, copies done %.2f, draws staged (incl. wait) %.2f, done %.2f\n",
-                !split ? "" : (phase == 0 ? " (first group's chunks)" : " (rest)"), tr_first, tr_queued, tr_copy, tr_draws, tr_front);
-    FTRY(dedup_error(err));
-#undef FTRY
-#undef FCUDA
-    if (total < 0 || (int64_t)total > cap) return SCDE_B200_OK;  // more rows than estimated: classic rebuild
-    t.n_rows = total;
-    if (last_phase) TRY(finish_table(ctx, t, &tm));
-    *done = true;
+    TRY(finish_table(ctx, t, &tm));
+    done->table = true;
     return SCDE_B200_OK;
 }
 
-static int diff_run_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, bool chunked_counts, ContractChoice k);
-
-extern "C" {
-
-int scde_b200_diff_upload(scde_b200_ctx *ctx, const scde_b200_diff_args *a, int32_t want_posteriors,
-                          scde_b200_diff_job **out) {
-    CHECK_CTX(ctx);
-    return diff_upload_impl(ctx, a, want_posteriors, out, false);
-}
-
-int scde_b200_diff_run(scde_b200_ctx *ctx, scde_b200_diff_job *j) {
-    CHECK_CTX(ctx);
-    return diff_run_impl(ctx, j, false, contraction_choice(ctx));
-}
-
-}  // extern "C"
-
-// chunked_counts: the count matrix is arriving in cell chunks on the copy stream (one-shot call)
-static int diff_run_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, bool chunked_counts, ContractChoice k) {
+// up, a: the one-shot call, whose count matrix is still arriving in chunks and whose draws are still to be made
+static int diff_run_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, ContractChoice k, CountUpload *up = nullptr,
+                         const scde_b200_diff_args *a = nullptr) {
     if (!j) return SCDE_B200_EINVAL;
     cudaStream_t st = ctx->stream;
     StageTimer &tm = j->timer;
@@ -2459,43 +2417,20 @@ static int diff_run_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, bool chunked
     const int ld = table_ld(K);
     SCDE_CUDA(cudaMemsetAsync(j->status.p, 0, 3 * sizeof(int32_t), st));
     int t_all = tm.begin(st);
-    bool front_done = false, joint0_done = false;
     const DrawSets sets{j->chunks.n_sets(), j->gene_set.p};
-    auto group_joint = [&](int i) {  // cells of one factor level, draws are local indices (R/functions.R:372-374)
-        const Joint jt{j->boot_ptr[i], j->D[i], j->ws->jp[i].p};
-        return run_joint(ctx, k, j->ws->table, j->cell_ids[i].p, j->n_group[i], &jt, 1, j->n_boot, sets, (double)j->n_boot,
-                         ld, j->ws->scr, j->status.p + i, &tm, true);
-    };
-    if (chunked_counts) {
-        TRY(front_chunked(ctx, j, k, 0, &front_done));
-        if (front_done && j->split_chunks > 0 && j->split_chunks < j->copy_chunks) {
-            // split front: every row of the first group's cells is built and within the capacity -- its joint runs
-            // while the rest of the count matrix is still arriving
-            TRY(group_joint(0));
-            joint0_done = true;
-            TRY(front_chunked(ctx, j, k, 1, &front_done));
-            if (!front_done) {  // the table is rebuilt below: row ids change, the first joint is repeated
-                joint0_done = false;
-                SCDE_CUDA(cudaMemsetAsync(j->ws->scr.total.p, 0, 5 * sizeof(unsigned long long), st));
-            }
-        }
-        if (!front_done && ctx->copy_stream) SCDE_CUDA(cudaStreamSynchronize(ctx->copy_stream));  // the counts must be resident
-    }
-    if (j->deferred_args) {  // not done by the chunked front (small problem or fallback)
-        const scde_b200_diff_args *da = j->deferred_args;
-        j->deferred_args = nullptr;
-        TRY(upload_draws(ctx, j, da));
-    }
+    FrontDone done;
+    if (up) TRY(front_chunked(ctx, j, k, *up, a, &done));
     j->rows_unchecked = false;
-    if (!front_done) {
-        // a repeated run of a resident job: the buffers of the last run are exactly large enough, no host round trip
-        const int64_t known = (!chunked_counts && k.kernel == Contraction::I8) ? j->known_rows : 0;
+    if (!done.table) {
+        // a repeated run of a resident job: the buffers of the last run are exactly large enough, no host round trip (a
+        // one-shot call's job is new: no known rows)
+        const int64_t known = k.kernel == Contraction::I8 ? j->known_rows : 0;
         TRY(index_from_counts(ctx, j->ws->table, j->ws->counts.p, G, 0, G, C, &tm, known));
         j->rows_unchecked = known > 0;
         TRY(fill_table(ctx, j->ws->table, diff_table(j->models, j->mag.p, K, k), &tm));
     }
     for (int i = 0; i < 2; ++i)
-        if (!(i == 0 && joint0_done)) TRY(group_joint(i));
+        if (!(i == 0 && done.joint0)) TRY(group_joint(ctx, j, k, i));
     // batch joints: all cells, composition-sampled draws are global cell ids (R/functions.R:355-357)
     if (j->has_batch) {
         // batch.models differ from models: the table rows are rebuilt from them (same row ids -- the counts have not
@@ -2561,7 +2496,7 @@ static int diff_download_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, const s
             j->rows_unchecked = false;
             if (err || total < 0 || (int64_t)total > j->known_rows) {
                 j->known_rows = 0;
-                TRY(diff_run_impl(ctx, j, false, k));
+                TRY(diff_run_impl(ctx, j, k));
                 SCDE_CUDA(cudaStreamSynchronize(st));
             } else {
                 j->ws->table.n_rows = total;
@@ -2572,7 +2507,7 @@ static int diff_download_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, const s
         bool rerun = false;
         TRY(read_status(j->status.p, f, 3, &rerun));
         if (rerun) {  // a multiplicity above 127: repeat the run on the FP64 contraction kernel
-            TRY(diff_run_impl(ctx, j, false, {Contraction::Tiled}));
+            TRY(diff_run_impl(ctx, j, {Contraction::Tiled}));
             SCDE_CUDA(cudaStreamSynchronize(st));
         }
     }
@@ -2611,6 +2546,34 @@ static int diff_download_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, const s
 
 extern "C" {
 
+int scde_b200_diff_upload(scde_b200_ctx *ctx, const scde_b200_diff_args *a, int32_t want_posteriors,
+                          scde_b200_diff_job **out) {
+    CHECK_CTX(ctx);
+    if (!out) return SCDE_B200_EINVAL;
+    *out = nullptr;
+    JobPtr j;
+    TRY(diff_upload_impl(ctx, a, want_posteriors, j));
+    TRY(upload_draws(ctx, j.get(), a));
+    // the counts shard, rows [gene_begin, gene_end) of every column, in one copy that has landed when the call returns
+    const WallClock clk;
+    SCDE_CUDA(j->ws->counts.ensure((size_t)j->G * j->C));
+    const double t_buf = clk.ms();
+    SCDE_CUDA(cudaMemcpy2DAsync(j->ws->counts.p, sizeof(int32_t) * j->G, a->counts + a->gene_begin,
+                                sizeof(int32_t) * (size_t)a->n_genes, sizeof(int32_t) * j->G, j->C, cudaMemcpyHostToDevice,
+                                ctx->stream));
+    SCDE_CUDA(cudaStreamSynchronize(ctx->stream));
+    if (ctx->opt.trace)
+        fprintf(stderr, "[scde_b200] upload: counts buffer %.2f ms, counts H2D (%.1f MB) %.2f ms\n", t_buf,
+                sizeof(int32_t) * (double)j->G * j->C / 1e6, clk.ms() - t_buf);
+    *out = j.release();
+    return SCDE_B200_OK;
+}
+
+int scde_b200_diff_run(scde_b200_ctx *ctx, scde_b200_diff_job *j) {
+    CHECK_CTX(ctx);
+    return diff_run_impl(ctx, j, contraction_choice(ctx));
+}
+
 int scde_b200_diff_download(scde_b200_ctx *ctx, scde_b200_diff_job *j, const scde_b200_diff_out *o, scde_b200_stats *stats) {
     CHECK_CTX(ctx);
     return diff_download_impl(ctx, j, o, stats, OutPlace{j ? j->G : 0, 0}, contraction_choice(ctx));
@@ -2630,25 +2593,21 @@ static int expression_difference_single(scde_b200_ctx *ctx, const scde_b200_diff
     CHECK_CTX(ctx);
     const ContractChoice k = contraction_choice(ctx);
     const int want_post = out->difference_posterior || out->adjusted_difference_posterior;
-    const bool trace = ctx->opt.trace != 0;  // host wall-clock of the three phases on stderr
-    auto now = [] { return std::chrono::steady_clock::now(); };
-    auto ms = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) {
-        return std::chrono::duration<double, std::milli>(b - a).count();
-    };
-    const auto t0 = now();
-    scde_b200_diff_job *job = nullptr;
-    int r = diff_upload_impl(ctx, args, want_post, &job, true);
-    if (r != SCDE_B200_OK) return r;
-    const auto t1 = now();
-    r = diff_run_impl(ctx, job, true, k);
-    if (r != SCDE_B200_OK && ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);
-    const auto t2 = now();
-    if (r == SCDE_B200_OK) r = diff_download_impl(ctx, job, out, stats, pl, k);
-    const auto t3 = now();
-    scde_b200_diff_free(ctx, job);
-    if (trace)
+    const WallClock clk;  // host wall-clock of the three phases on stderr (trace)
+    JobPtr job;
+    TRY(diff_upload_impl(ctx, args, want_post, job));
+    // the small uploads above share the one H2D copy engine with these 1.2 GB and would queue behind them
+    CountUpload up(ctx);
+    TRY(up.start(*job, args->counts + args->gene_begin, args->n_genes));
+    const double t_up = clk.ms();
+    int r = diff_run_impl(ctx, job.get(), k, &up, args);
+    const double t_run = clk.ms();
+    if (r == SCDE_B200_OK) r = diff_download_impl(ctx, job.get(), out, stats, pl, k);
+    const double t_down = clk.ms();
+    job.reset();
+    if (ctx->opt.trace)
         fprintf(stderr, "[scde_b200] expression_difference (device %d): upload %.2f ms, run (queued) %.2f ms, download (incl. wait) %.2f ms, free %.2f ms\n",
-                ctx->device, ms(t0, t1), ms(t1, t2), ms(t2, t3), ms(t3, now()));
+                ctx->device, t_up, t_run - t_up, t_down - t_run, clk.ms() - t_down);
     return r;
 }
 

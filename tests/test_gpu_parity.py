@@ -531,6 +531,27 @@ def test_one_shot_call_split_front_overflow_after_first_joint():
     _assert_same(one, two)
 
 
+def test_one_shot_call_split_front_error_after_first_joint():
+    """split front with a negative count in a cell of the second group: the first group's rows are clean, so its joint
+    runs, and the rest of the front finds the bad count.  The call raises, and it leaves the context usable: the same call
+    on clean counts equals the job path bit for bit, and the job that follows is not refused as another live job"""
+    w = synth.make_workload(3, n_genes=200, n_cells=640, seed=23)
+    counts = np.array(w.counts, dtype=np.int32, order="F")
+    bad = counts.copy(order="F")
+    bad[57, 500] = -3
+    mm, lt, sq = api.pack_models(w.models)
+    x, y = w.prior["x"].to_numpy(), w.prior["y"].to_numpy()
+    codes = np.asarray(w.groups.codes, dtype=np.int32)
+    assert np.all(codes[:320] == 0) and np.all(codes[320:] == 1)
+    zi = api._zero_index(api.fold_change_grid(x), 0.0)
+    ctx = _lib.Context(0)
+    with pytest.raises(_lib.ScdeB200Error, match="negative count"):
+        api.expression_difference_call(ctx, bad, mm, x, y, codes, 100, 1, zero_index=zi, local_theta=lt, sqlogit=sq,
+                                       joint_posteriors=True)
+    one, two = _call_and_job(ctx, w, counts)
+    _assert_same(one, two)
+
+
 def test_one_shot_call_group_layouts(ctx):
     """where the first group's cells lie decides whether the front is split: interleaved groups (no split), the first
     group in the trailing cells (no split), a short first group (split after a quarter), cells outside both groups"""
