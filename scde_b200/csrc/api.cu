@@ -462,15 +462,11 @@ struct Joint {
     double *jp_dev;
 };
 
-// The tcgen05 contraction of joints[0 .. n_joints) (two: joints over the same cells and entry lists with their own draws)
-// whose operands run_joint has prepared.  The launches raise bits in *status (read_status).
-// prune (DESIGN.md 4.3): before each launch a bound pass and a decision find the (gene, piece) items the soft-max cannot
-// see; the contraction and the soft-max then skip them.  prune_stats (or NULL): launch_prune_items' four counters.
-int contract_joint_i8(scde_b200_ctx *ctx, const LpTable &t, const GeneLists &lists, JointScratch &scr, int n_w_rows,
-                      int n_boot, const DrawSets &sets, double scale, const Joint *joints, int n_joints, int ld_jp,
-                      int hot_rank, int32_t *status, StageTimer *tm, bool prune, unsigned long long *prune_stats) {
-    cudaStream_t st = ctx->stream;
-    const int passes = (n_boot + WP_TILED - 1) / WP_TILED;
+// The launch arguments of the tcgen05 contraction over the fixed-point table t (its planes, row ranges, K and sentinel)
+// and the entry lists, with the context's kernel options; the launches raise bits in *status (read_status).  Draw sets,
+// ld_jp, the epilogue counters and pruning's buffers are left to the caller.
+ContractI8Args i8_args(const scde_b200_ctx *ctx, const LpTable &t, const GeneLists &lists, int n_w_rows, int n_boot,
+                       double scale, int32_t *status) {
     ContractI8Args q{};
     q.qtable = t.q.p;
     q.ldq = q_row_bytes(t.K);
@@ -478,19 +474,31 @@ int contract_joint_i8(scde_b200_ctx *ctx, const LpTable &t, const GeneLists &lis
     q.lists = lists;
     q.n_w_rows = n_w_rows;
     q.n_boot = n_boot;
-    q.gene_set = sets.gene_set;
-    q.set_w8 = (int64_t)passes * n_w_rows * Q_WB;
-    q.set_z = (int64_t)passes * WP_TILED * KP_TILED;
     q.scale = scale;
     q.sentinel = t.sentinel;
     q.K = t.K;
-    q.ld_jp = ld_jp;
     q.err = status;
-    q.dbg = nullptr;
     q.item_order = ctx->opt.item_order;
-    q.hot_rank = hot_rank;
+    q.hot_rank = ctx->opt.hot_rank;
     q.cold_evict_first = ctx->opt.cold_evict_first;
     q.ring_stages = ctx->opt.ring_stages;
+    return q;
+}
+
+// The tcgen05 contraction of joints[0 .. n_joints) (two: joints over the same cells and entry lists with their own draws)
+// whose operands run_joint has prepared.  The launches raise bits in *status (read_status).
+// prune (DESIGN.md 4.3): before each launch a bound pass and a decision find the (gene, piece) items the soft-max cannot
+// see; the contraction and the soft-max then skip them.  prune_stats (or NULL): launch_prune_items' four counters.
+int contract_joint_i8(scde_b200_ctx *ctx, const LpTable &t, const GeneLists &lists, JointScratch &scr, int n_w_rows,
+                      int n_boot, const DrawSets &sets, double scale, const Joint *joints, int n_joints, int ld_jp,
+                      int32_t *status, StageTimer *tm, bool prune, unsigned long long *prune_stats) {
+    cudaStream_t st = ctx->stream;
+    const int passes = (n_boot + WP_TILED - 1) / WP_TILED;
+    ContractI8Args q = i8_args(ctx, t, lists, n_w_rows, n_boot, scale, status);
+    q.gene_set = sets.gene_set;
+    q.set_w8 = (int64_t)passes * n_w_rows * Q_WB;
+    q.set_z = (int64_t)passes * WP_TILED * KP_TILED;
+    q.ld_jp = ld_jp;
     if (ctx->opt.epilogue_timing) {
         SCDE_CUDA(ctx->epi_dbg.ensure(3));
         SCDE_CUDA(cudaMemsetAsync(ctx->epi_dbg.p, 0, 3 * sizeof(unsigned long long), st));
@@ -682,7 +690,7 @@ int run_joint(scde_b200_ctx *ctx, ContractChoice k, const LpTable &t, const int3
     if (!i8)
         return contract_joint_fp64(ctx, k.kernel, t, lists, scr, zb ? scr.Z[0].p : nullptr, n_w_rows, n_boot, sets, scale,
                                    joints[0].jp_dev, ld_jp, tm);
-    return contract_joint_i8(ctx, t, lists, scr, n_w_rows, n_boot, sets, scale, joints, n_joints, ld_jp, hot_rank, status, tm,
+    return contract_joint_i8(ctx, t, lists, scr, n_w_rows, n_boot, sets, scale, joints, n_joints, ld_jp, status, tm,
                              t.plan.bounds && ctx->opt.prune_pieces && n_list >= PRUNE_MIN_CELLS,
                              count_entries ? scr.total.p + 1 : nullptr);
 }
@@ -805,6 +813,48 @@ TableRequest diff_table(const ModelSet &ms, const double *mag_dev, int K, Contra
     return r;
 }
 
+// Caller-given unique-count lists of n cells: cell c's counts are flat[off[c], off[c + 1]), with off[0] = 0 and off
+// monotone.  strict (the probes): the counts of every cell distinct, ascending and >= 0, and at least one row.
+int check_lists(const char *who, const int32_t *flat, const int32_t *off, int n, bool strict) {
+    if (off[0] != 0) {
+        set_error("%s: ucl_offsets[0] must be 0", who);
+        return SCDE_B200_EINVAL;
+    }
+    for (int c = 0; c < n; ++c) {
+        if (off[c + 1] < off[c]) {
+            set_error("%s: ucl_offsets not monotone at cell %d", who, c);
+            return SCDE_B200_EINVAL;
+        }
+        if (strict)
+            for (int r = off[c]; r < off[c + 1]; ++r)
+                if (flat[r] < 0 || (r > off[c] && flat[r] <= flat[r - 1])) {
+                    set_error("%s: the counts of cell %d are not distinct, ascending and >= 0", who, c);
+                    return SCDE_B200_EINVAL;
+                }
+    }
+    if (strict && off[n] < 1) {
+        set_error("%s: no table rows", who);
+        return SCDE_B200_EINVAL;
+    }
+    return SCDE_B200_OK;
+}
+
+// The table of a per-call entry point, over lists check_lists has accepted: the C cells' models (C x 12, column-major),
+// the K magnitudes of the grid and the lists uploaded to ms, mag and t, then the table r asks for (r.K, r.clamp_n and the
+// flags are the caller's; r.models and r.mag are set here).  ms and mag stay with the table: a rebuild reuses r.
+int list_table(scde_b200_ctx *ctx, LpTable &t, ModelSet &ms, DBuf<double> &mag, TableRequest &r, const double *models, int C,
+               int local_theta, int sqlogit, const double *magnitudes, const int32_t *flat, const int32_t *off) {
+    cudaStream_t st = ctx->stream;
+    t.n_rows = off[C];
+    TRY(upload_models(ms, models, C, local_theta, sqlogit, st));
+    TRY(upload(mag, magnitudes, (size_t)r.K, st));
+    TRY(upload(t.row_off, off, (size_t)C + 1, st));
+    TRY(upload(t.row_x, flat, (size_t)t.n_rows, st));
+    r.models = &ms;
+    r.mag = mag.p;
+    return fill_table(ctx, t, r, nullptr);
+}
+
 int workspace_busy(const scde_b200_ctx *ctx) {
     if (!ctx->ws_busy) return SCDE_B200_OK;
     set_error("another expression_difference job is alive on this context (free it first)");
@@ -861,6 +911,35 @@ int launch_ratio_passes(const RatioPasses &r, bool has_batch, cudaStream_t st) {
     return SCDE_B200_OK;
 }
 
+// The two posterior matrices of a per-call ratio summary (G x n, column-major on the host), uploaded gene-major, and the
+// call's geometry: nout = 2n - 1 ratio points; a holds the matrices, ld, n_genes, n and ld_post, the caller the rest.
+struct RatioInput {
+    DBuf<double> staging, m1, m2;
+    int nout = 0;
+    RatioArgs a{};
+};
+
+int upload_ratio_input(scde_b200_ctx *ctx, const double *m1, const double *m2, int G, int n, RatioInput &in) {
+    cudaStream_t st = ctx->stream;
+    const int ld = round_up(n, 8);
+    const size_t sz = (size_t)G * n;
+    SCDE_CUDA(in.staging.ensure(sz));
+    SCDE_CUDA(in.m1.ensure((size_t)G * ld));
+    SCDE_CUDA(in.m2.ensure((size_t)G * ld));
+    SCDE_CUDA(cudaMemcpyAsync(in.staging.p, m1, sizeof(double) * sz, cudaMemcpyHostToDevice, st));
+    SCDE_CUDA(launch_transpose_in(in.staging.p, G, n, in.m1.p, ld, st));
+    SCDE_CUDA(cudaMemcpyAsync(in.staging.p, m2, sizeof(double) * sz, cudaMemcpyHostToDevice, st));
+    SCDE_CUDA(launch_transpose_in(in.staging.p, G, n, in.m2.p, ld, st));
+    in.nout = 2 * n - 1;
+    in.a.p1 = in.m1.p;
+    in.a.p2 = in.m2.p;
+    in.a.ld = ld;
+    in.a.n_genes = G;
+    in.a.n = n;
+    in.a.ld_post = round_up(in.nout, 8);
+    return SCDE_B200_OK;
+}
+
 // Where a job's per-gene results go in the caller's (column-major) output matrices: row `row0` of matrices with `ld`
 // rows.  A single-device call writes whole matrices (ld = the job's genes, row0 = 0); the shards of a multi-device call
 // write their gene range of the same buffers.
@@ -877,6 +956,19 @@ int download_summary(cudaStream_t st, int G, const int32_t *idx, const double *z
                                     sizeof(int32_t) * (size_t)G, sizeof(int32_t) * (size_t)G, 3, cudaMemcpyDeviceToHost, st));
     if (z_dst)
         SCDE_CUDA(cudaMemcpyAsync(z_dst + block * pl.ld + pl.row0, z, sizeof(double) * (size_t)G, cudaMemcpyDeviceToHost, st));
+    return SCDE_B200_OK;
+}
+
+// [G][ld_src] gene-major device matrix -> rows pl.row0.. of a column-major host matrix with pl.ld rows, transposed through
+// tbuf; returns once the copy is done
+int download_matrix(scde_b200_ctx *ctx, DBuf<double> &tbuf, int G, const double *src, int ld_src, int cols, double *dst,
+                    OutPlace pl) {
+    cudaStream_t st = ctx->stream;
+    SCDE_CUDA(tbuf.ensure((size_t)G * cols));
+    SCDE_CUDA(launch_transpose_out(src, ld_src, G, cols, tbuf.p, st));
+    SCDE_CUDA(cudaMemcpy2DAsync(dst + pl.row0, sizeof(double) * (size_t)pl.ld, tbuf.p, sizeof(double) * (size_t)G,
+                                sizeof(double) * (size_t)G, cols, cudaMemcpyDeviceToHost, st));
+    SCDE_CUDA(cudaStreamSynchronize(st));
     return SCDE_B200_OK;
 }
 
@@ -1249,17 +1341,12 @@ int scde_b200_cell_table(scde_b200_ctx *ctx, const double *model_row12, const in
     }
     cudaStream_t st = ctx->stream;
     LpTable t;
-    t.n_rows = n_counts;
     ModelSet ms;
     DBuf<double> d_mag;
-    TRY(upload_models(ms, model_row12, 1, local_theta, square_logit_conc, st));
-    TRY(upload(d_mag, magnitudes, (size_t)n_grid, st));
-    int32_t off[2] = {0, n_counts};
-    TRY(upload(t.row_off, off, 2, st));
-    TRY(upload(t.row_x, unique_counts, (size_t)n_counts, st));
-    TableRequest r{&ms, d_mag.p, n_grid, n_cells_for_clamp};
+    const int32_t off[2] = {0, n_counts};
+    TableRequest r{nullptr, nullptr, n_grid, n_cells_for_clamp};
     r.modes = true;
-    TRY(fill_table(ctx, t, r, nullptr));
+    TRY(list_table(ctx, t, ms, d_mag, r, model_row12, 1, local_theta, square_logit_conc, magnitudes, unique_counts, off));
     if (n_counts > 0) {
         SCDE_CUDA(cudaMemcpy2DAsync(out, sizeof(double) * n_grid, t.table.p, sizeof(double) * t.ld, sizeof(double) * n_grid,
                                     n_counts, cudaMemcpyDeviceToHost, st));
@@ -1287,7 +1374,7 @@ int scde_b200_probe_table_bounds(scde_b200_ctx *ctx, const double *models, int32
                                  int32_t *zero_row_out, int32_t *based_out, double *zero_rows_out, int8_t *qbound_out) {
     CHECK_CTX(ctx);
     if (!models || !ucl_flat || !ucl_offsets || !magnitudes || !q_out || !row_range_out || !zero_row_out || !based_out ||
-        !zero_rows_out || n_cells < 1 || n_grid < 1 || n_cells_for_clamp < 1 || ucl_offsets[0] != 0) {
+        !zero_rows_out || n_cells < 1 || n_grid < 1 || n_cells_for_clamp < 1) {
         set_error("probe_table: bad arguments");
         return SCDE_B200_EINVAL;
     }
@@ -1295,34 +1382,16 @@ int scde_b200_probe_table_bounds(scde_b200_ctx *ctx, const double *models, int32
         set_error("probe_table: no fixed-point table for %d grid points (at most %d)", n_grid, Q_MAX_K);
         return SCDE_B200_EINVAL;
     }
-    for (int c = 0; c < n_cells; ++c) {
-        if (ucl_offsets[c + 1] < ucl_offsets[c]) {
-            set_error("probe_table: ucl_offsets not monotone at cell %d", c);
-            return SCDE_B200_EINVAL;
-        }
-        for (int r = ucl_offsets[c]; r < ucl_offsets[c + 1]; ++r)
-            if (ucl_flat[r] < 0 || (r > ucl_offsets[c] && ucl_flat[r] <= ucl_flat[r - 1])) {
-                set_error("probe_table: the counts of cell %d are not distinct, ascending and >= 0", c);
-                return SCDE_B200_EINVAL;
-            }
-    }
-    if (ucl_offsets[n_cells] < 1) {
-        set_error("probe_table: no table rows");
-        return SCDE_B200_EINVAL;
-    }
+    TRY(check_lists("probe_table", ucl_flat, ucl_offsets, n_cells, true));
     cudaStream_t st = ctx->stream;
     LpTable t;
-    t.n_rows = ucl_offsets[n_cells];
     ModelSet ms;
     DBuf<double> d_mag;
-    TRY(upload_models(ms, models, n_cells, local_theta, square_logit_conc, st));
-    TRY(upload(d_mag, magnitudes, (size_t)n_grid, st));
-    TRY(upload(t.row_off, ucl_offsets, (size_t)n_cells + 1, st));
-    TRY(upload(t.row_x, ucl_flat, (size_t)t.n_rows, st));
-    TableRequest r{&ms, d_mag.p, n_grid, n_cells_for_clamp};
+    TableRequest r{nullptr, nullptr, n_grid, n_cells_for_clamp};
     r.zero_base = r.fixed_point = r.probe = true;
     r.bounds = qbound_out != nullptr;
-    TRY(fill_table(ctx, t, r, nullptr));
+    TRY(list_table(ctx, t, ms, d_mag, r, models, n_cells, local_theta, square_logit_conc, magnitudes, ucl_flat,
+                   ucl_offsets));
     if (!t.plan.planes) {
         set_error("probe_table: the table was built without fixed-point planes");
         return SCDE_B200_EINVAL;
@@ -1349,31 +1418,23 @@ int scde_b200_probe_table_bounds(scde_b200_ctx *ctx, const double *models, int32
 }
 
 // --------------------------------------------------------------------------------------------
-static int log_boot_impl(scde_b200_ctx *ctx, const double *models, int32_t n_cells, const int32_t *ucl_flat,
-                           const int32_t *ucl_offsets, const int32_t *uci, int32_t n_genes, const double *magnitudes,
-                           int32_t n_grid, int32_t n_boot, const int32_t *boot_idx, int32_t D, int32_t return_individual,
-                           int32_t local_theta, int32_t square_logit_conc, int32_t ensemble, int32_t modes_flag,
-                           int32_t post_flag, double *jp, double *modes, double *post, ContractChoice k, bool *rerun) {
+// The joint posterior of the cells (or the ensemble), and with modes_flag / post_flag their posterior modes and individual
+// posteriors.  When the tcgen05 status word asks for the FP64 kernel, the table is rebuilt in FP64 from the same uploads
+// and the joint runs again on the tiled FP64 kernel, before anything is copied out.
+static int log_boot(scde_b200_ctx *ctx, const double *models, int32_t n_cells, const int32_t *ucl_flat,
+                    const int32_t *ucl_offsets, const int32_t *uci, int32_t n_genes, const double *magnitudes,
+                    int32_t n_grid, int32_t n_boot, const int32_t *boot_idx, int32_t D, int32_t local_theta,
+                    int32_t square_logit_conc, int32_t ensemble, int32_t modes_flag, int32_t post_flag, double *jp,
+                    double *modes, double *post) {
     cudaStream_t st = ctx->stream;
-    (void)return_individual;
-    *rerun = false;
     if (!models || !ucl_flat || !ucl_offsets || !uci || !magnitudes || !jp || n_cells < 1 || n_genes < 0 || n_grid < 1 ||
         n_boot < 0) {
         set_error("log_boot_posterior: bad arguments");
         return SCDE_B200_EINVAL;
     }
-    if (ucl_offsets[0] != 0) {
-        set_error("ucl_offsets[0] must be 0");
-        return SCDE_B200_EINVAL;
-    }
-    for (int c = 0; c < n_cells; ++c) {
-        if (ucl_offsets[c + 1] < ucl_offsets[c]) {
-            set_error("ucl_offsets not monotone at cell %d", c);
-            return SCDE_B200_EINVAL;
-        }
-        const int nu = ucl_offsets[c + 1] - ucl_offsets[c];
-        TRY(validate_index(uci + (size_t)c * n_genes, (size_t)n_genes, 0, nu, "uci"));
-    }
+    TRY(check_lists("log_boot_posterior", ucl_flat, ucl_offsets, n_cells, false));
+    for (int c = 0; c < n_cells; ++c)
+        TRY(validate_index(uci + (size_t)c * n_genes, (size_t)n_genes, 0, ucl_offsets[c + 1] - ucl_offsets[c], "uci"));
     if (modes_flag && !modes) {
         set_error("modes requested but the output pointer is NULL");
         return SCDE_B200_EINVAL;
@@ -1383,55 +1444,62 @@ static int log_boot_impl(scde_b200_ctx *ctx, const double *models, int32_t n_cel
         return SCDE_B200_EINVAL;
     }
     if (n_genes == 0) return SCDE_B200_OK;
+    const ContractChoice k = contraction_choice(ctx);
     LpTable t;
     t.n_genes = n_genes;
     t.ld_ridx = n_cells;
-    t.n_rows = ucl_offsets[n_cells];
     const double minlogprob = -DBL_MAX / n_cells / 1.1;  // src/jpmatLogBoot.cpp:127,372
     ModelSet ms;
     DBuf<double> d_mag, d_jp, d_out, d_rs;
     DBuf<int32_t> d_uci, d_boot, status;
     SCDE_CUDA(status.ensure(1));
     SCDE_CUDA(cudaMemsetAsync(status.p, 0, sizeof(int32_t), st));
-    TRY(upload_models(ms, models, n_cells, local_theta, square_logit_conc, st));
-    TRY(upload(d_mag, magnitudes, (size_t)n_grid, st));
-    TRY(upload(t.row_off, ucl_offsets, (size_t)n_cells + 1, st));
-    TRY(upload(t.row_x, ucl_flat, (size_t)t.n_rows, st));
-    TRY(upload(d_uci, uci, (size_t)n_genes * n_cells, st));
-    SCDE_CUDA(t.ridx.ensure((size_t)n_genes * n_cells));
-    SCDE_CUDA(launch_uci_to_ridx(d_uci.p, n_genes, n_cells, t.row_off.p, t.ridx.p, t.ld_ridx, st));
-    TableRequest r{&ms, d_mag.p, n_grid, D > n_cells ? D : n_cells};
+    TableRequest r{nullptr, nullptr, n_grid, D > n_cells ? D : n_cells};
     r.zero_base = !post_flag && !ensemble;
     r.fixed_point = k.kernel == Contraction::I8 && n_boot > 0;
     r.modes = modes_flag != 0;
-    TRY(fill_table(ctx, t, r, nullptr));
+    TRY(list_table(ctx, t, ms, d_mag, r, models, n_cells, local_theta, square_logit_conc, magnitudes, ucl_flat,
+                   ucl_offsets));
+    TRY(upload(d_uci, uci, (size_t)n_genes * n_cells, st));
+    SCDE_CUDA(t.ridx.ensure((size_t)n_genes * n_cells));
+    SCDE_CUDA(launch_uci_to_ridx(d_uci.p, n_genes, n_cells, t.row_off.p, t.ridx.p, t.ld_ridx, st));
     const int ld_jp = t.ld;
     SCDE_CUDA(d_jp.ensure((size_t)n_genes * ld_jp));
+    std::vector<int32_t> gen;
+    int nb = n_boot, dd = D;
+    double scale = (double)n_boot;
+    if (!ensemble && n_boot == 0) {  // plain product over all cells, src/jpmatLogBoot.cpp:239-249
+        gen.resize(n_cells);
+        for (int c = 0; c < n_cells; ++c) gen[c] = c;
+        boot_idx = gen.data();
+        nb = 1;
+        dd = n_cells;
+        scale = 1.0;
+    }
     JointScratch scr;
+    auto joint = [&](ContractChoice kc) {
+        const Joint jt{d_boot.p, dd, d_jp.p};
+        return run_joint(ctx, kc, t, nullptr, n_cells, &jt, 1, nb, {}, scale, ld_jp, scr, status.p, nullptr, false);
+    };
     if (ensemble) {
         SCDE_CUDA(d_rs.ensure((size_t)t.n_rows));
         SCDE_CUDA(launch_ensemble(t.table.p, t.ld, t.ridx.p, t.ld_ridx, n_cells, n_genes, n_grid, d_jp.p, ld_jp, d_rs.p,
                                   t.n_rows, st));
     } else {
-        std::vector<int32_t> gen;
-        int nb = n_boot, dd = D;
-        double scale = (double)n_boot;
-        if (n_boot == 0) {  // plain product over all cells, src/jpmatLogBoot.cpp:239-249
-            gen.resize(n_cells);
-            for (int c = 0; c < n_cells; ++c) gen[c] = c;
-            boot_idx = gen.data();
-            nb = 1;
-            dd = n_cells;
-            scale = 1.0;
-        }
         TRY(validate_index(boot_idx, (size_t)nb * dd, 0, n_cells, "boot_idx"));
         TRY(upload(d_boot, boot_idx, (size_t)nb * dd, st));
-        const Joint jt{d_boot.p, dd, d_jp.p};
-        TRY(run_joint(ctx, k, t, nullptr, n_cells, &jt, 1, nb, {}, scale, ld_jp, scr, status.p, nullptr, false));
+        TRY(joint(k));
     }
-    SCDE_CUDA(d_out.ensure((size_t)n_genes * n_grid));
-    SCDE_CUDA(launch_transpose_out(d_jp.p, ld_jp, n_genes, n_grid, d_out.p, st));
-    SCDE_CUDA(cudaMemcpyAsync(jp, d_out.p, sizeof(double) * (size_t)n_genes * n_grid, cudaMemcpyDeviceToHost, st));
+    SCDE_CUDA(cudaStreamSynchronize(st));
+    int32_t f = 0;
+    bool rerun = false;
+    TRY(read_status(status.p, &f, 1, &rerun));
+    if (rerun) {  // a cell drawn more than 127 times in one randomization, or "log 0" rows only the FP64 kernel adds
+        r.fixed_point = false;
+        TRY(fill_table(ctx, t, r, nullptr));
+        TRY(joint({Contraction::Tiled}));
+    }
+    TRY(download_matrix(ctx, d_out, n_genes, d_jp.p, ld_jp, n_grid, jp, OutPlace{n_genes, 0}));
     if (modes_flag) {
         DBuf<double> d_modes;
         SCDE_CUDA(d_modes.ensure((size_t)n_genes * n_cells));
@@ -1448,25 +1516,7 @@ static int log_boot_impl(scde_b200_ctx *ctx, const double *models, int32_t n_cel
         SCDE_CUDA(cudaMemcpyAsync(post, d_post.p, sizeof(double) * np, cudaMemcpyDeviceToHost, st));
         SCDE_CUDA(cudaStreamSynchronize(st));
     }
-    SCDE_CUDA(cudaStreamSynchronize(st));
-    int32_t f = 0;
-    return read_status(status.p, &f, 1, rerun);
-}
-
-static int log_boot_common(scde_b200_ctx *ctx, const double *models, int32_t n_cells, const int32_t *ucl_flat,
-                           const int32_t *ucl_offsets, const int32_t *uci, int32_t n_genes, const double *magnitudes,
-                           int32_t n_grid, int32_t n_boot, const int32_t *boot_idx, int32_t D, int32_t return_individual,
-                           int32_t local_theta, int32_t square_logit_conc, int32_t ensemble, int32_t modes_flag,
-                           int32_t post_flag, double *jp, double *modes, double *post) {
-    bool rerun = false;
-    TRY(log_boot_impl(ctx, models, n_cells, ucl_flat, ucl_offsets, uci, n_genes, magnitudes, n_grid, n_boot, boot_idx, D,
-                      return_individual, local_theta, square_logit_conc, ensemble, modes_flag, post_flag, jp, modes, post,
-                      contraction_choice(ctx), &rerun));
-    if (!rerun) return SCDE_B200_OK;
-    // a cell drawn more than 127 times in one randomization: outside the int8 operand range
-    return log_boot_impl(ctx, models, n_cells, ucl_flat, ucl_offsets, uci, n_genes, magnitudes, n_grid, n_boot, boot_idx, D,
-                         return_individual, local_theta, square_logit_conc, ensemble, modes_flag, post_flag, jp, modes, post,
-                         {Contraction::Tiled}, &rerun);
+    return SCDE_B200_OK;
 }
 
 int scde_b200_log_boot_posterior(scde_b200_ctx *ctx, const double *models, int32_t n_cells, const int32_t *ucl_flat,
@@ -1486,8 +1536,8 @@ int scde_b200_log_boot_posterior(scde_b200_ctx *ctx, const double *models, int32
     }
     const int mf = (return_individual == 1 || return_individual == 3);
     const int pf = (return_individual == 2 || return_individual == 3);
-    return log_boot_common(ctx, models, n_cells, ucl_flat, ucl_offsets, uci, n_genes, magnitudes, n_grid, n_boot, boot_idx,
-                           n_cells, return_individual, local_theta, square_logit_conc, ensemble, mf, pf, jp, modes, post);
+    return log_boot(ctx, models, n_cells, ucl_flat, ucl_offsets, uci, n_genes, magnitudes, n_grid, n_boot, boot_idx, n_cells,
+                    local_theta, square_logit_conc, ensemble, mf, pf, jp, modes, post);
 }
 
 int scde_b200_log_boot_batch_posterior(scde_b200_ctx *ctx, const double *models, int32_t n_cells,
@@ -1522,8 +1572,8 @@ int scde_b200_log_boot_batch_posterior(scde_b200_ctx *ctx, const double *models,
     }
     const int mf = (return_individual == 1);  // src/jpmatLogBoot.cpp:441,455,501
     const int pf = (return_individual == 2 || return_individual == 3);
-    return log_boot_common(ctx, models, n_cells, ucl_flat, ucl_offsets, uci, n_genes, magnitudes, n_grid, n_boot, boot_idx, D,
-                           return_individual, local_theta, square_logit_conc, 0, mf, pf, jp, modes, post);
+    return log_boot(ctx, models, n_cells, ucl_flat, ucl_offsets, uci, n_genes, magnitudes, n_grid, n_boot, boot_idx, D,
+                    local_theta, square_logit_conc, 0, mf, pf, jp, modes, post);
 }
 
 // --------------------------------------------------------------------------------------------
@@ -1570,11 +1620,7 @@ static int jpmat_common(scde_b200_ctx *ctx, const double *matl, int n_mat, int n
     } else {
         SCDE_CUDA(cudaMemsetAsync(d_jp.p, 0, sizeof(double) * (size_t)n_rows * t.ld, st));
     }
-    SCDE_CUDA(d_out.ensure(sz));
-    SCDE_CUDA(launch_transpose_out(d_jp.p, t.ld, n_rows, n_cols, d_out.p, st));
-    SCDE_CUDA(cudaMemcpyAsync(jp, d_out.p, sizeof(double) * sz, cudaMemcpyDeviceToHost, st));
-    SCDE_CUDA(cudaStreamSynchronize(st));
-    return SCDE_B200_OK;
+    return download_matrix(ctx, d_out, n_rows, d_jp.p, t.ld, n_cols, jp, OutPlace{n_rows, 0});
 }
 
 int scde_b200_jpmat_log_boot(scde_b200_ctx *ctx, const double *matl, int32_t n_mat, int32_t n_rows, int32_t n_cols,
@@ -1627,32 +1673,13 @@ int scde_b200_mat_slide_mult(scde_b200_ctx *ctx, const double *m1, const double 
         return SCDE_B200_EINVAL;
     }
     if (n_rows == 0) return SCDE_B200_OK;
-    cudaStream_t st = ctx->stream;
-    const int nout = 2 * n - 1, ld = round_up(n, 8), ldo = round_up(nout, 8);
-    DBuf<double> d_in, d1, d2, d_raw, d_out;
-    const size_t sz = (size_t)n_rows * n;
-    SCDE_CUDA(d_in.ensure(sz));
-    SCDE_CUDA(d1.ensure((size_t)n_rows * ld));
-    SCDE_CUDA(d2.ensure((size_t)n_rows * ld));
-    SCDE_CUDA(cudaMemcpyAsync(d_in.p, m1, sizeof(double) * sz, cudaMemcpyHostToDevice, st));
-    SCDE_CUDA(launch_transpose_in(d_in.p, n_rows, n, d1.p, ld, st));
-    SCDE_CUDA(cudaMemcpyAsync(d_in.p, m2, sizeof(double) * sz, cudaMemcpyHostToDevice, st));
-    SCDE_CUDA(launch_transpose_in(d_in.p, n_rows, n, d2.p, ld, st));
-    SCDE_CUDA(d_raw.ensure((size_t)n_rows * ldo));
-    RatioArgs a{};
-    a.p1 = d1.p;
-    a.p2 = d2.p;
-    a.ld = ld;
-    a.n_genes = n_rows;
-    a.n = n;
-    a.ld_post = ldo;
-    a.raw = d_raw.p;
-    SCDE_CUDA(launch_ratio_summary(a, st));
-    SCDE_CUDA(d_out.ensure((size_t)n_rows * nout));
-    SCDE_CUDA(launch_transpose_out(d_raw.p, ldo, n_rows, nout, d_out.p, st));
-    SCDE_CUDA(cudaMemcpyAsync(out, d_out.p, sizeof(double) * (size_t)n_rows * nout, cudaMemcpyDeviceToHost, st));
-    SCDE_CUDA(cudaStreamSynchronize(st));
-    return SCDE_B200_OK;
+    RatioInput in;
+    DBuf<double> d_raw, d_out;
+    TRY(upload_ratio_input(ctx, m1, m2, n_rows, n, in));
+    SCDE_CUDA(d_raw.ensure((size_t)n_rows * in.a.ld_post));
+    in.a.raw = d_raw.p;
+    SCDE_CUDA(launch_ratio_summary(in.a, ctx->stream));
+    return download_matrix(ctx, d_out, n_rows, d_raw.p, in.a.ld_post, in.nout, out, OutPlace{n_rows, 0});
 }
 
 int scde_b200_ratio_posterior_summary(scde_b200_ctx *ctx, const double *pmat1, const double *pmat2, int32_t n_genes,
@@ -1666,43 +1693,27 @@ int scde_b200_ratio_posterior_summary(scde_b200_ctx *ctx, const double *pmat1, c
     if (n_genes == 0) return SCDE_B200_OK;
     TRY(validate_index(zero_index, (size_t)n_zero, 1, 2 * n, "zero_index"));
     cudaStream_t st = ctx->stream;
-    const int nout = 2 * n - 1, ld = round_up(n, 8), ldo = round_up(nout, 8);
-    DBuf<double> d_in, d1, d2, d_prior, d_post, d_out, d_z;
+    RatioInput in;
+    DBuf<double> d_prior, d_post, d_out, d_z;
     DBuf<int32_t> d_zi, d_idx;
-    const size_t sz = (size_t)n_genes * n;
-    SCDE_CUDA(d_in.ensure(sz));
-    SCDE_CUDA(d1.ensure((size_t)n_genes * ld));
-    SCDE_CUDA(d2.ensure((size_t)n_genes * ld));
-    SCDE_CUDA(cudaMemcpyAsync(d_in.p, pmat1, sizeof(double) * sz, cudaMemcpyHostToDevice, st));
-    SCDE_CUDA(launch_transpose_in(d_in.p, n_genes, n, d1.p, ld, st));
-    SCDE_CUDA(cudaMemcpyAsync(d_in.p, pmat2, sizeof(double) * sz, cudaMemcpyHostToDevice, st));
-    SCDE_CUDA(launch_transpose_in(d_in.p, n_genes, n, d2.p, ld, st));
+    TRY(upload_ratio_input(ctx, pmat1, pmat2, n_genes, n, in));
     if (prior_y) TRY(upload(d_prior, prior_y, (size_t)n, st));
     TRY(upload(d_zi, zero_index, (size_t)n_zero, st));
     SCDE_CUDA(d_idx.ensure((size_t)3 * n_genes));
     SCDE_CUDA(d_z.ensure((size_t)n_genes));
-    if (posterior) SCDE_CUDA(d_post.ensure((size_t)n_genes * ldo));
-    RatioArgs a{};
-    a.p1 = d1.p;
-    a.p2 = d2.p;
-    a.ld = ld;
-    a.n_genes = n_genes;
-    a.n = n;
+    if (posterior) SCDE_CUDA(d_post.ensure((size_t)n_genes * in.a.ld_post));
+    RatioArgs &a = in.a;
     a.prior = prior_y ? d_prior.p : nullptr;
     a.zero_index = d_zi.p;
     a.n_zero = n_zero;
     a.idx = d_idx.p;
     a.z = d_z.p;
     a.post = posterior ? d_post.p : nullptr;
-    a.ld_post = ldo;
     SCDE_CUDA(launch_ratio_summary(a, st));
     if (idx) SCDE_CUDA(cudaMemcpyAsync(idx, d_idx.p, sizeof(int32_t) * 3 * (size_t)n_genes, cudaMemcpyDeviceToHost, st));
     if (z) SCDE_CUDA(cudaMemcpyAsync(z, d_z.p, sizeof(double) * (size_t)n_genes, cudaMemcpyDeviceToHost, st));
-    if (posterior) {
-        SCDE_CUDA(d_out.ensure((size_t)n_genes * nout));
-        SCDE_CUDA(launch_transpose_out(d_post.p, ldo, n_genes, nout, d_out.p, st));
-        SCDE_CUDA(cudaMemcpyAsync(posterior, d_out.p, sizeof(double) * (size_t)n_genes * nout, cudaMemcpyDeviceToHost, st));
-    }
+    if (posterior)
+        return download_matrix(ctx, d_out, n_genes, d_post.p, a.ld_post, in.nout, posterior, OutPlace{n_genes, 0});
     SCDE_CUDA(cudaStreamSynchronize(st));
     return SCDE_B200_OK;
 }
@@ -1903,13 +1914,15 @@ int scde_b200_probe_prune_i8(scde_b200_ctx *ctx, const int8_t *qtable, int32_t n
     TRY(validate_index(lst_row, (size_t)n_genes * ld_lst, 0, n_rows, "lst_row"));
     TRY(validate_index(lst_cell, (size_t)n_genes * ld_lst, 0, n_w_rows, "lst_cell"));
     cudaStream_t st = ctx->stream;
-    DBuf<int8_t> d_q, d_w;
+    LpTable t;  // the caller's fixed-point table: its planes, row ranges (or none) and bound rows
+    t.K = n_grid;
+    t.sentinel = -1.0e300;
+    DBuf<int8_t> d_w;
     DBuf<int32_t> d_row, d_cell, d_len, status;
-    DBuf<uint32_t> d_rr, d_sr;
+    DBuf<uint32_t> d_sr;
     DBuf<double> d_t;
-    const int ldq = q_row_bytes(n_grid);
-    TRY(upload(d_q, qtable, (size_t)n_rows * ldq, st));
-    if (row_range) TRY(upload(d_rr, row_range, (size_t)n_rows, st));
+    TRY(upload(t.q, qtable, (size_t)n_rows * q_row_bytes(n_grid), st));
+    if (row_range) TRY(upload(t.qrange, row_range, (size_t)n_rows, st));
     TRY(upload(d_w, w8, (size_t)n_w_rows * Q_WB, st));
     TRY(upload(d_row, lst_row, (size_t)n_genes * ld_lst, st));
     TRY(upload(d_cell, lst_cell, (size_t)n_genes * ld_lst, st));
@@ -1920,32 +1933,20 @@ int scde_b200_probe_prune_i8(scde_b200_ctx *ctx, const int8_t *qtable, int32_t n
     SCDE_CUDA(cudaMemsetAsync(d_t.p, 0, sizeof(double) * nt, st));
     SCDE_CUDA(status.ensure(1));
     SCDE_CUDA(cudaMemsetAsync(status.p, 0, sizeof(int32_t), st));
-    ContractI8Args q{};
-    q.qtable = d_q.p;
-    q.ldq = ldq;
-    q.row_range = row_range ? d_rr.p : nullptr;
-    q.lists = GeneLists{d_row.p, d_cell.p, d_len.p, nullptr, ld_lst};
-    q.n_w_rows = n_w_rows;
-    q.n_boot = WP_TILED;
-    q.scale = 1.0;
-    q.sentinel = -1.0e300;
-    q.K = n_grid;
-    q.ld_jp = 0;
-    q.err = status.p;
-    q.item_order = ctx->opt.item_order;
+    // one pass of 104 boots, no output matrix, no L2 hints
+    ContractI8Args q = i8_args(ctx, t, GeneLists{d_row.p, d_cell.p, d_len.p, nullptr, ld_lst}, n_w_rows, WP_TILED, 1.0,
+                               status.p);
     q.hot_rank = -1;
     q.cold_evict_first = 0;
-    q.ring_stages = ctx->opt.ring_stages;
     I8Side side{d_w.p, nullptr, d_t.p, d_sr.p, nullptr, nullptr, 0};
     SCDE_CUDA(launch_sentinel_ranges(q, 0, n_genes, side, st));
-    DBuf<int8_t> d_qb;
     DBuf<double> d_z, d_zb, d_lb, d_ub;
     DBuf<int32_t> d_items, d_nlive;
     DBuf<uint8_t> d_live;
     if (qbound) {  // the decision of the pruned contraction, with its bounds; T itself is contracted unpruned
-        TRY(upload(d_qb, qbound, (size_t)n_rows * Q_BW, st));
+        TRY(upload(t.qb, qbound, (size_t)n_rows * Q_BW, st));
         if (z) TRY(upload(d_z, z, (size_t)WP_TILED * KP_TILED, st));
-        q.qbound = d_qb.p;
+        q.qbound = t.qb.p;
         SCDE_CUDA(d_zb.ensure(prune_zb_doubles(1, WP_TILED)));
         SCDE_CUDA(d_lb.ensure((size_t)n_genes * WP_TILED));
         SCDE_CUDA(d_ub.ensure((size_t)n_genes * WP_TILED * 4));
@@ -2466,18 +2467,6 @@ static int diff_run_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, ContractChoi
     return SCDE_B200_OK;
 }
 
-// [G][ld_src] gene-major device matrix -> rows row0.. of a column-major host matrix with pl.ld rows
-static int download_matrix(scde_b200_ctx *ctx, DiffWorkspace *ws, int G, const double *src, int ld_src, int cols, double *dst,
-                           OutPlace pl) {
-    cudaStream_t st = ctx->stream;
-    SCDE_CUDA(ws->tbuf.ensure((size_t)G * cols));
-    SCDE_CUDA(launch_transpose_out(src, ld_src, G, cols, ws->tbuf.p, st));
-    SCDE_CUDA(cudaMemcpy2DAsync(dst + pl.row0, sizeof(double) * (size_t)pl.ld, ws->tbuf.p, sizeof(double) * (size_t)G,
-                                sizeof(double) * (size_t)G, cols, cudaMemcpyDeviceToHost, st));
-    SCDE_CUDA(cudaStreamSynchronize(st));
-    return SCDE_B200_OK;
-}
-
 static int diff_download_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, const scde_b200_diff_out *o,
                               scde_b200_stats *stats, OutPlace pl, ContractChoice k) {
     if (!j || !j->ran) {
@@ -2519,25 +2508,26 @@ static int diff_download_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, const s
         }
         SCDE_CUDA(cudaStreamSynchronize(st));
         for (int i = 0; i < 2; ++i) {
-            if (o->joint_posteriors[i]) TRY(download_matrix(ctx, j->ws, j->G, j->ws->jp[i].p, ld, K, o->joint_posteriors[i], pl));
+            if (o->joint_posteriors[i])
+                TRY(download_matrix(ctx, j->ws->tbuf, j->G, j->ws->jp[i].p, ld, K, o->joint_posteriors[i], pl));
             if (j->has_batch && o->batch_joint_posteriors[i])
-                TRY(download_matrix(ctx, j->ws, j->G, j->ws->jp[2 + i].p, ld, K, o->batch_joint_posteriors[i], pl));
+                TRY(download_matrix(ctx, j->ws->tbuf, j->G, j->ws->jp[2 + i].p, ld, K, o->batch_joint_posteriors[i], pl));
         }
         if (o->difference_posterior) {
             if (!j->ws->post.p) {
                 set_error("difference_posterior requested but the job was uploaded without want_posteriors");
                 return SCDE_B200_EINVAL;
             }
-            TRY(download_matrix(ctx, j->ws, j->G, j->ws->post.p, ldo, nout, o->difference_posterior, pl));
+            TRY(download_matrix(ctx, j->ws->tbuf, j->G, j->ws->post.p, ldo, nout, o->difference_posterior, pl));
         }
         if (j->has_batch && o->batch_difference_posterior)
-            TRY(download_matrix(ctx, j->ws, j->G, j->ws->bpost.p, ldo, nout, o->batch_difference_posterior, pl));
+            TRY(download_matrix(ctx, j->ws->tbuf, j->G, j->ws->bpost.p, ldo, nout, o->batch_difference_posterior, pl));
         if (j->has_batch && o->adjusted_difference_posterior) {
             if (!j->ws->apost.p) {
                 set_error("adjusted posterior requested but the job was uploaded without want_posteriors");
                 return SCDE_B200_EINVAL;
             }
-            TRY(download_matrix(ctx, j->ws, j->G, j->ws->apost.p, lda, nadj, o->adjusted_difference_posterior, pl));
+            TRY(download_matrix(ctx, j->ws->tbuf, j->G, j->ws->apost.p, lda, nadj, o->adjusted_difference_posterior, pl));
         }
     }
     SCDE_CUDA(cudaStreamSynchronize(st));
@@ -2954,10 +2944,10 @@ int shard_contrasts(DatasetShard &sh, const ContrastPlan &p, const scde_b200_con
         for (int c = c0; c < c0 + n && p.want_post; ++c) {
             const size_t k = (size_t)(c - c0);
             if (o->difference_posterior)
-                TRY(download_matrix(ctx, ws, G, ws->post.p + k * G * ldo, ldo, nout, o->difference_posterior + (size_t)c * N * nout,
-                                    OutPlace{N, sh.g0}));
+                TRY(download_matrix(ctx, ws->tbuf, G, ws->post.p + k * G * ldo, ldo, nout,
+                                    o->difference_posterior + (size_t)c * N * nout, OutPlace{N, sh.g0}));
             if (p.has_batch && o->adjusted_difference_posterior)
-                TRY(download_matrix(ctx, ws, G, ws->apost.p + k * G * lda, lda, nadj,
+                TRY(download_matrix(ctx, ws->tbuf, G, ws->apost.p + k * G * lda, lda, nadj,
                                     o->adjusted_difference_posterior + (size_t)c * N * nadj, OutPlace{N, sh.g0}));
         }
     }
@@ -2972,7 +2962,7 @@ int shard_contrasts(DatasetShard &sh, const ContrastPlan &p, const scde_b200_con
     }
     if (o->joint_posteriors)
         for (int s = 0; s < n_slots; ++s)
-            TRY(download_matrix(ctx, ws, G, sh.bank.p + s * slot_sz, ld, K,
+            TRY(download_matrix(ctx, ws->tbuf, G, sh.bank.p + s * slot_sz, ld, K,
                                 o->joint_posteriors + (size_t)p.slot_group[s] * N * K, pl));
     SCDE_CUDA(cudaStreamSynchronize(st));
     return collect_stats(tm, ws, stats);

@@ -44,7 +44,8 @@ def _log_boot(ctx, w, bi):
 @pytest.mark.parametrize("call", [_one_shot, _resident_job, _log_boot], ids=["one_shot", "resident_job", "log_boot"])
 def test_multiplicity_fallback_keeps_options_and_equals_fp64_kernel(ctx, call):
     """every draw of a group of 150 cells hits its first cell: a multiplicity of 150 does not fit the int8 operand, so
-    the whole call (log_boot) or the whole run (two-group job) is repeated on the FP64 DMMA kernel"""
+    the joint (log_boot, on its table rebuilt in FP64) or the whole run (two-group job) is repeated on the FP64 DMMA
+    kernel"""
     w = synth.make_workload(3, n_genes=150, n_cells=150 if call is _log_boot else 640, seed=2)
     bi = np.zeros((N_BOOT, 150), dtype=np.int32)
     res = {}
