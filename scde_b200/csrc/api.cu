@@ -5,6 +5,7 @@
 #include "common.cuh"
 #include "hostmath.h"
 
+#include <algorithm>
 #include <cfloat>
 #include <cmath>
 #include <cstdarg>
@@ -1031,18 +1032,6 @@ int check_draw_chunks(int32_t n, bool explicit_draws, const char *who) {
     return SCDE_B200_OK;
 }
 
-// the seeds of all draw sets over genes [0, N), in chunk order
-std::vector<int32_t> chunk_seeds(int N, int n, int seed) {
-    if (!(n > 1 && N > n)) return {seed};
-    std::vector<int32_t> v(n);
-    for (int i = 0; i < n; ++i) {
-        int b = 0, e = 0;
-        shard_range(N, n, i, &b, &e);
-        v[i] = seed + b;
-    }
-    return v;
-}
-
 DrawChunks draw_chunks_of(int N, int n, int seed, int g0, int g1) {
     DrawChunks d;
     if (!(n > 1 && N > n)) {
@@ -1103,6 +1092,141 @@ int parallel_for(int n, F f) {
             g_err = msg[i];
             return rc[i];
         }
+    return SCDE_B200_OK;
+}
+
+// The joints of one differential-expression call, on the host (DESIGN.md §11, §12).  Group joint i runs over its cells
+// cells[cell_off[i], cell_off[i + 1]); the batch joints run over all C cells, in pairs (2q, 2q + 1; an odd last one alone).
+// Each joint reads one draw block; a block holds n_boot x D draws per draw set.  Status words: group joint i has word i,
+// batch pair q word n_groups() + q.
+struct DrawBlock {
+    int D = 0;                       // draws per randomization
+    bool batch = false;              // global cell ids from the batch pools following comp; else local indices of D cells
+    std::vector<int32_t> comp;
+    const int32_t *given = nullptr;  // the caller's draws (one set) instead of generated ones
+};
+
+struct JointPlan {
+    int C = 0, n_boot = 0;
+    int N = 0, draw_chunks = 0, seed = 1;  // the call's genes, and what its draw sets follow
+    DrawChunks sets;                       // the sets of the plan's genes
+    BatchPools pools;
+    std::vector<DrawBlock> blocks;
+    std::vector<int32_t> cells;
+    std::vector<int64_t> cell_off{0};
+    std::vector<int> group_block, batch_block;  // joint -> its block
+
+    JointPlan() = default;
+    JointPlan(int C, int n_boot, int N, int draw_chunks, int seed, int g0, int g1)
+        : C(C), n_boot(n_boot), N(N), draw_chunks(draw_chunks), seed(seed), sets(sets_of(g0, g1)) {}
+    int n_groups() const { return (int)group_block.size(); }
+    int n_words() const { return n_groups() + ((int)batch_block.size() + 1) / 2; }
+    DrawChunks sets_of(int g0, int g1) const { return draw_chunks_of(N, draw_chunks, seed, g0, g1); }
+    size_t per_set(int b) const { return (size_t)n_boot * blocks[b].D; }
+    // where block b starts when every block holds n sets (b = blocks.size(): the total)
+    size_t block_off(int b, int n) const {
+        size_t o = 0;
+        for (int i = 0; i < b; ++i) o += (size_t)n * per_set(i);
+        return o;
+    }
+};
+
+// Every (block, set) of p into dst, block b's sets at dst + p.block_off(b, all sets), one task each on parallel_for
+// (src/jpmatLogBoot.cpp:221,254-257 / :467-481).  A block of the caller's draws is validated; stage_given copies it to
+// dst as well (the mapped pinned staging), otherwise upload_draws reads it from the caller's array.
+int generate_draws(const JointPlan &p, int32_t *dst, bool stage_given) {
+    const int S = p.sets.n_sets(), L = (int)p.pools.off.size() - 1;
+    std::vector<std::pair<int, int>> tasks;  // (block, set); set -1 copies the caller's draws
+    for (int b = 0; b < (int)p.blocks.size(); ++b) {
+        const DrawBlock &k = p.blocks[b];
+        if (!k.given) {
+            for (int s = 0; s < S; ++s) tasks.emplace_back(b, s);
+            continue;
+        }
+        if (k.D > 0)
+            TRY(validate_index(k.given, p.per_set(b), 0, k.batch ? p.C : k.D, k.batch ? "batch boot_idx" : "boot_idx"));
+        if (stage_given) tasks.emplace_back(b, -1);
+    }
+    return parallel_for((int)tasks.size(), [&](int t) -> int {
+        const int b = tasks[t].first, s = tasks[t].second;
+        const DrawBlock &k = p.blocks[b];
+        int32_t *out = dst + p.block_off(b, S);
+        if (s < 0) {
+            memcpy(out, k.given, sizeof(int32_t) * p.per_set(b));
+            return SCDE_B200_OK;
+        }
+        out += s * p.per_set(b);
+        if (!k.batch) return scde_b200_boot_indices(p.sets.seeds[s], k.D, p.n_boot, out);
+        return scde_b200_batch_boot_indices(p.sets.seeds[s], L, p.pools.off.data(), p.pools.pool.data(), k.comp.data(),
+                                            p.n_boot, out);
+    });
+}
+
+// A plan's joints on one device: the group joints' cells, the draw sets of the device's genes (block b at
+// draws + block_off(b, sets.n)) with their gene_set, the status words and where each joint writes
+struct JointDevice {
+    DBuf<int32_t> cells, buf, gene_set, status;
+    const int32_t *draws = nullptr;  // buf.p, or the mapped pinned staging the W build reads in place
+    DrawSets sets;
+    std::vector<double *> jp;        // joint -> its output, G x ld (group joints, then batch joints)
+};
+
+// the cells of p and the gene_set of the device's sets dc on the device (queued: the host vectors must outlive the copies)
+int place_joints(scde_b200_ctx *ctx, const JointPlan &p, const DrawChunks &dc, JointDevice &d) {
+    cudaStream_t st = ctx->stream;
+    TRY(upload(d.cells, p.cells.data(), p.cells.size(), st));
+    if (dc.n_sets() > 1) TRY(upload(d.gene_set, dc.gene_set.data(), dc.gene_set.size(), st));
+    d.sets = DrawSets{dc.n_sets(), dc.n_sets() > 1 ? d.gene_set.p : nullptr};
+    SCDE_CUDA(d.status.ensure((size_t)p.n_words()));
+    return SCDE_B200_OK;
+}
+
+// the sets dc of every block of p, one copy per block: from src (generate_draws' layout over all of p's sets) or from the
+// caller's array (queued: both must outlive the copies)
+int upload_draws(scde_b200_ctx *ctx, const JointPlan &p, const DrawChunks &dc, const int32_t *src, JointDevice &d) {
+    const int nb = (int)p.blocks.size(), n = dc.n_sets();
+    const size_t skip = (size_t)(dc.first - p.sets.first);
+    SCDE_CUDA(d.buf.ensure(p.block_off(nb, n)));
+    for (int b = 0; b < nb; ++b) {
+        const size_t len = (size_t)n * p.per_set(b);
+        const int32_t *from =
+            p.blocks[b].given ? p.blocks[b].given : src + p.block_off(b, p.sets.n_sets()) + skip * p.per_set(b);
+        if (len)
+            SCDE_CUDA(cudaMemcpyAsync(d.buf.p + p.block_off(b, n), from, sizeof(int32_t) * len, cudaMemcpyHostToDevice,
+                                      ctx->stream));
+    }
+    d.draws = d.buf.p;
+    return SCDE_B200_OK;
+}
+
+// The group joints of p whose status word mask selects, on the table t for the kernel k
+int run_group_joints(scde_b200_ctx *ctx, ContractChoice k, const LpTable &t, const JointPlan &p, const JointDevice &d,
+                     const std::vector<bool> &mask, JointScratch &scr, StageTimer *tm, bool count_entries) {
+    for (int i = 0; i < p.n_groups(); ++i) {
+        if (!mask[i]) continue;
+        const int b = p.group_block[i];
+        const Joint jt{d.draws + p.block_off(b, d.sets.n), p.blocks[b].D, d.jp[i]};
+        TRY(run_joint(ctx, k, t, d.cells.p + p.cell_off[i], (int)(p.cell_off[i + 1] - p.cell_off[i]), &jt, 1, p.n_boot,
+                      d.sets, (double)p.n_boot, t.ld, scr, d.status.p + i, tm, count_entries));
+    }
+    return SCDE_B200_OK;
+}
+
+// The batch pairs of p whose status word mask selects
+int run_batch_joints(scde_b200_ctx *ctx, ContractChoice k, const LpTable &t, const JointPlan &p, const JointDevice &d,
+                     const std::vector<bool> &mask, JointScratch &scr, StageTimer *tm, bool count_entries) {
+    const int ng = p.n_groups(), nb = (int)p.batch_block.size();
+    for (int q = 0; 2 * q < nb; ++q) {
+        if (!mask[ng + q]) continue;
+        const int n = nb - 2 * q < 2 ? 1 : 2;
+        Joint js[2];
+        for (int i = 0; i < n; ++i) {
+            const int b = p.batch_block[2 * q + i];
+            js[i] = Joint{d.draws + p.block_off(b, d.sets.n), p.blocks[b].D, d.jp[ng + 2 * q + i]};
+        }
+        TRY(run_joint(ctx, k, t, nullptr, p.C, js, n, p.n_boot, d.sets, (double)p.n_boot, t.ld, scr, d.status.p + ng + q,
+                      tm, count_entries));
+    }
     return SCDE_B200_OK;
 }
 
@@ -1982,30 +2106,22 @@ int scde_b200_probe_prune_i8(scde_b200_ctx *ctx, const int8_t *qtable, int32_t n
 struct scde_b200_diff_job {
     int G = 0, C = 0, K = 0, n_boot = 0, n_levels = 0;
     int want_post = 0, has_batch = 0;
-    int n_group[2] = {0, 0};
     int n_zero = 1;
     DiffWorkspace *ws = nullptr;
     scde_b200_ctx *owner = nullptr;
     ModelSet models;
     ModelSet bmodels;           // batch.models when they differ from models (else empty)
     DBuf<double> mag, prior_y;
-    DBuf<int32_t> cell_ids[2];  // group cell lists
-    DBuf<int32_t> boot[4];      // draws of each joint: one block of n_boot x D[i] per draw set
-    int D[4] = {0, 0, 0, 0};
-    DrawChunks chunks;          // the draw sets of the job's genes
-    DBuf<int32_t> gene_set;     // chunks.gene_set on the device
+    JointPlan joints;           // groups 0 and 1, with a batch factor the two batch joints (jp[0 .. 3])
+    JointDevice dj;
     DBuf<int32_t> zi, zi_adj;
     DBuf<int32_t> idx, bidx, aidx;
     DBuf<double> z, bz, az;
-    DBuf<int32_t> status;       // tcgen05 status words of the last run: group 0, group 1, the batch joints
     StageTimer timer;
     bool ran = false;
     int64_t known_rows = 0;          // table rows of the last completed run of this job (0: unknown): the next run needs no
                                      // size read-back -- same counts, same rows
     bool rows_unchecked = false;     // the last run used known_rows as the capacity; download verifies it
-    const int32_t *boot_ptr[4] = {nullptr, nullptr, nullptr, nullptr};  // draws as the device reads them
-    std::vector<int32_t> ids[2];                 // cells of the two groups
-    std::unique_ptr<int32_t[]> gen[4];           // generated draws (resident job), alive until their uploads have completed
 };
 
 // A job owned by a scope: released as scde_b200_diff_free releases it, on every return
@@ -2020,85 +2136,31 @@ struct WallClock {
     double ms() const { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count(); }
 };
 
-// Bootstrap draws of the group joints (local indices) and, with a batch factor, of the composition-sampled joints (global
-// cell ids): the caller's, or generated from the seed (src/jpmatLogBoot.cpp:221,254-257 / :467-481).  The uploads are
-// queued on the context stream; the host vectors live in the job.
-// pinned: the draws go to the context's mapped pinned staging and are read in place (one-shot call with a split front:
-// an H2D copy would queue behind the count matrix on the copy engine, and the first joint starts before that has landed).
-int upload_draws(scde_b200_ctx *ctx, scde_b200_diff_job *j, const scde_b200_diff_args *a, bool pinned = false) {
-    cudaStream_t st = ctx->stream;
-    const int C = j->C;
-    const int S = j->chunks.n_sets();  // draw sets per joint (a->boot_idx are NULL when S > 1)
-    const int n_joints = j->has_batch ? 4 : 2;
-    // draws per joint and the caller's explicit draws, validated
-    BatchPools bp;
-    std::vector<int32_t> comp[2];
-    for (int i = 0; i < 2; ++i) j->D[i] = j->n_group[i];
-    if (j->has_batch) {
-        TRY(batch_pools(a->batch, C, a->n_batch_levels, bp));
-        for (int i = 0; i < 2; ++i)
-            j->D[2 + i] = batch_composition(a->batch, a->n_batch_levels, j->ids[i].data(), j->ids[i].size(), comp[i]);
+// The job's draws, generated where the device reads them.  pinned: into the context's mapped pinned staging, read in
+// place (one-shot call with a split front: an H2D copy would queue behind the count matrix on the copy engine, and the
+// first joint starts before that has landed).  Otherwise into a host buffer that is uploaded.  Neither destination is
+// zero-filled first, so the one-shot call pays neither a zero-fill nor a copy of the draws before its first joint.
+static int job_draws(scde_b200_ctx *ctx, scde_b200_diff_job *j, bool pinned = false) {
+    const JointPlan &p = j->joints;
+    const size_t total = p.block_off((int)p.blocks.size(), p.sets.n_sets());
+    if (!pinned) {
+        std::unique_ptr<int32_t[]> host(new int32_t[total]);
+        TRY(generate_draws(p, host.get(), false));
+        TRY(upload_draws(ctx, p, p.sets, host.get(), j->dj));
+        SCDE_CUDA(cudaStreamSynchronize(ctx->stream));  // the caller's (or this) host array has been read
+        return SCDE_B200_OK;
     }
-    for (int i = 0; i < n_joints; ++i)
-        if (a->boot_idx[i] && j->D[i] > 0)
-            TRY(validate_index(a->boot_idx[i], (size_t)a->n_boot * j->D[i], 0, i < 2 ? j->D[i] : C,
-                               i < 2 ? "boot_idx" : "batch boot_idx"));
-    // Destinations: the mapped pinned staging (read in place by the W build) or, for an upload, host buffers that are
-    // not zero-filled first.  The generators write straight into them, one (joint, set) per task on parallel host
-    // threads, so the one-shot call pays neither a zero-fill nor a copy of the draws before its first joint.
-    int32_t *dst[4] = {nullptr, nullptr, nullptr, nullptr};
+    if (total > ctx->h_draws_cap) {
+        if (ctx->h_draws) cudaFreeHost(ctx->h_draws);
+        ctx->h_draws = nullptr;
+        ctx->h_draws_cap = 0;
+        SCDE_CUDA(cudaHostAlloc((void **)&ctx->h_draws, sizeof(int32_t) * total, cudaHostAllocMapped));
+        ctx->h_draws_cap = total;
+    }
     int32_t *dev = nullptr;
-    if (pinned) {
-        size_t total = 0;
-        for (int i = 0; i < n_joints; ++i) total += (size_t)S * a->n_boot * j->D[i];
-        if (total > ctx->h_draws_cap) {
-            if (ctx->h_draws) cudaFreeHost(ctx->h_draws);
-            ctx->h_draws = nullptr;
-            ctx->h_draws_cap = 0;
-            SCDE_CUDA(cudaHostAlloc((void **)&ctx->h_draws, sizeof(int32_t) * total, cudaHostAllocMapped));
-            ctx->h_draws_cap = total;
-        }
-        SCDE_CUDA(cudaHostGetDevicePointer((void **)&dev, ctx->h_draws, 0));
-        size_t off = 0;
-        for (int i = 0; i < n_joints; ++i) {
-            dst[i] = ctx->h_draws + off;
-            j->boot_ptr[i] = dev + off;
-            off += (size_t)S * a->n_boot * j->D[i];
-        }
-    } else {
-        for (int i = 0; i < n_joints; ++i)
-            if (!a->boot_idx[i]) {
-                j->gen[i].reset(new int32_t[(size_t)S * a->n_boot * j->D[i]]);
-                dst[i] = j->gen[i].get();
-            }
-    }
-    std::vector<std::pair<int, int>> tasks;  // (joint, set); an explicit set is one copy task (pinned) or none
-    for (int i = 0; i < n_joints; ++i) {
-        if (a->boot_idx[i]) {
-            if (pinned) tasks.emplace_back(i, -1);
-            continue;
-        }
-        for (int s = 0; s < S; ++s) tasks.emplace_back(i, s);
-    }
-    const std::vector<int32_t> &seeds = j->chunks.seeds;
-    TRY(parallel_for((int)tasks.size(), [&](int t) -> int {
-        const int i = tasks[t].first, s = tasks[t].second;
-        const size_t per = (size_t)a->n_boot * j->D[i];
-        if (s < 0) {
-            memcpy(dst[i], a->boot_idx[i], sizeof(int32_t) * per);
-            return SCDE_B200_OK;
-        }
-        int32_t *out = dst[i] + s * per;
-        if (i < 2) return scde_b200_boot_indices(seeds[s], j->n_group[i], a->n_boot, out);
-        return scde_b200_batch_boot_indices(seeds[s], a->n_batch_levels, bp.off.data(), bp.pool.data(), comp[i - 2].data(),
-                                            a->n_boot, out);
-    }));
-    if (pinned) return SCDE_B200_OK;
-    for (int i = 0; i < n_joints; ++i) {
-        TRY(upload(j->boot[i], a->boot_idx[i] ? a->boot_idx[i] : dst[i], (size_t)S * a->n_boot * j->D[i], st));
-        j->boot_ptr[i] = j->boot[i].p;
-    }
-    SCDE_CUDA(cudaStreamSynchronize(st));  // the caller's (or the job's) host arrays have been read
+    SCDE_CUDA(cudaHostGetDevicePointer((void **)&dev, ctx->h_draws, 0));
+    TRY(generate_draws(p, ctx->h_draws, true));
+    j->dj.draws = dev;
     return SCDE_B200_OK;
 }
 
@@ -2167,8 +2229,8 @@ struct CountUpload {
     int start(const scde_b200_diff_job &j, const int32_t *counts_host, int64_t ld_host) {
         const int G = j.G, C = j.C;
         const int n = ctx->opt.count_chunks > 0 ? ctx->opt.count_chunks : default_options().count_chunks;
-        bounds = count_chunk_bounds(C, n, ctx->opt.split_front ? j.ids[0].back() : -1, ctx->opt.uniform_chunks != 0,
-                                    &split);
+        const int last0 = j.joints.cells[j.joints.cell_off[1] - 1];  // the first group's last cell
+        bounds = count_chunk_bounds(C, n, ctx->opt.split_front ? last0 : -1, ctx->opt.uniform_chunks != 0, &split);
         SCDE_CUDA(j.ws->counts.ensure((size_t)G * C));
         if (!ctx->copy_stream) SCDE_CUDA(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
         while ((int)ctx->copy_events.size() < chunks() + 1) {
@@ -2212,6 +2274,35 @@ static int gene_range(const scde_b200_diff_args *a, int *g0, int *g1) {
     return SCDE_B200_OK;
 }
 
+// The joints of a two-group call, into p (its draw sets already set): groups 0 and 1 of a->group and, with a batch factor,
+// the two batch joints of their compositions (R/functions.R:355-357), each with its own block, the caller's draws where
+// given.
+// Equal sizes or compositions are not merged: the two batch joints share one launch of the tcgen05 kernel either way.
+static int job_joints(const scde_b200_diff_args *a, bool has_batch, JointPlan &p) {
+    const int C = a->n_cells;
+    for (int i = 0; i < 2; ++i) {
+        for (int c = 0; c < C; ++c)
+            if (a->group[c] == i) p.cells.push_back(c);
+        p.cell_off.push_back((int64_t)p.cells.size());
+        p.group_block.push_back(i);
+        p.blocks.push_back(DrawBlock{(int)(p.cell_off[i + 1] - p.cell_off[i]), false, {}, a->boot_idx[i]});
+    }
+    if (p.blocks[0].D == 0 || p.blocks[1].D == 0) {
+        set_error("both groups need at least one cell");
+        return SCDE_B200_EINVAL;
+    }
+    if (has_batch) {
+        TRY(batch_pools(a->batch, C, a->n_batch_levels, p.pools));
+        for (int i = 0; i < 2; ++i) {
+            p.batch_block.push_back(2 + i);
+            p.blocks.push_back(DrawBlock{0, true, {}, a->boot_idx[2 + i]});
+            p.blocks.back().D = batch_composition(a->batch, a->n_batch_levels, p.cells.data() + p.cell_off[i],
+                                                  (size_t)(p.cell_off[i + 1] - p.cell_off[i]), p.blocks.back().comp);
+        }
+    }
+    return SCDE_B200_OK;
+}
+
 // A job with everything on the device but its count matrix and its draws, which the caller uploads: the resident job in
 // one copy, the one-shot call in chunks overlapped with the table build
 static int diff_upload_impl(scde_b200_ctx *ctx, const scde_b200_diff_args *a, int32_t want_posteriors, JobPtr &out) {
@@ -2226,14 +2317,9 @@ static int diff_upload_impl(scde_b200_ctx *ctx, const scde_b200_diff_args *a, in
     TRY(check_draw_chunks(a->draw_chunks, a->boot_idx[0] || a->boot_idx[1] || a->boot_idx[2] || a->boot_idx[3],
                           "expression_difference"));
     const int G = g1 - g0, C = a->n_cells, K = a->n_grid;
-    std::vector<int32_t> ids[2];
-    for (int c = 0; c < C; ++c)
-        if (a->group[c] == 0 || a->group[c] == 1) ids[a->group[c]].push_back(c);
-    if (ids[0].empty() || ids[1].empty()) {
-        set_error("both groups need at least one cell");
-        return SCDE_B200_EINVAL;
-    }
     const bool has_batch = a->batch != nullptr && a->n_batch_levels > 1;
+    JointPlan joints(C, a->n_boot, a->n_genes, a->draw_chunks, a->seed, g0, g1);
+    TRY(job_joints(a, has_batch, joints));
     if (a->n_zero != 1 && a->n_zero != a->n_genes) {
         set_error("n_zero must be 1 or n_genes");
         return SCDE_B200_EINVAL;
@@ -2261,14 +2347,8 @@ static int diff_upload_impl(scde_b200_ctx *ctx, const scde_b200_diff_args *a, in
     TRY(upload(j->prior_y, a->prior_y, (size_t)K, st));
     const std::vector<double> mag = grid_magnitudes(a->prior_x, K);
     TRY(upload(j->mag, mag.data(), (size_t)K, st));
-    for (int i = 0; i < 2; ++i) {
-        j->n_group[i] = (int)ids[i].size();
-        TRY(upload(j->cell_ids[i], ids[i].data(), ids[i].size(), st));
-    }
-    j->ids[0] = ids[0];
-    j->ids[1] = ids[1];
-    j->chunks = draw_chunks_of(a->n_genes, a->draw_chunks, a->seed, g0, g1);
-    if (j->chunks.n_sets() > 1) TRY(upload(j->gene_set, j->chunks.gene_set.data(), j->chunks.gene_set.size(), st));
+    j->joints = std::move(joints);
+    TRY(place_joints(ctx, j->joints, j->joints.sets, j->dj));
     {
         const std::vector<int32_t> zi = zero_slice(a->zero_index, a->n_zero, g0, G);
         TRY(validate_index(zi.data(), zi.size(), 1, 2 * K, "zero_index"));
@@ -2281,10 +2361,12 @@ static int diff_upload_impl(scde_b200_ctx *ctx, const scde_b200_diff_args *a, in
         SCDE_CUDA(cudaStreamSynchronize(st));
     }
     const int ld = table_ld(K), nout = 2 * K - 1, ldo = round_up(nout, 8), nadj = 2 * nout - 1, lda = round_up(nadj, 8);
-    for (int i = 0; i < (has_batch ? 4 : 2); ++i) SCDE_CUDA(j->ws->jp[i].ensure((size_t)G * ld));
+    for (int i = 0; i < (has_batch ? 4 : 2); ++i) {
+        SCDE_CUDA(j->ws->jp[i].ensure((size_t)G * ld));
+        j->dj.jp.push_back(j->ws->jp[i].p);
+    }
     SCDE_CUDA(j->idx.ensure((size_t)3 * G));
     SCDE_CUDA(j->z.ensure((size_t)G));
-    SCDE_CUDA(j->status.ensure(3));
     if (want_posteriors || has_batch) SCDE_CUDA(j->ws->post.ensure((size_t)G * ldo));
     if (has_batch) {
         SCDE_CUDA(j->ws->bpost.ensure((size_t)G * ldo));
@@ -2297,14 +2379,6 @@ static int diff_upload_impl(scde_b200_ctx *ctx, const scde_b200_diff_args *a, in
     SCDE_CUDA(cudaStreamSynchronize(st));
     out = std::move(j);
     return SCDE_B200_OK;
-}
-
-// the joint of group i: cells of one factor level, draws are local indices (R/functions.R:372-374)
-static int group_joint(scde_b200_ctx *ctx, scde_b200_diff_job *j, ContractChoice k, int i) {
-    const Joint jt{j->boot_ptr[i], j->D[i], j->ws->jp[i].p};
-    return run_joint(ctx, k, j->ws->table, j->cell_ids[i].p, j->n_group[i], &jt, 1, j->n_boot,
-                     DrawSets{j->chunks.n_sets(), j->gene_set.p}, (double)j->n_boot, table_ld(j->K), j->ws->scr,
-                     j->status.p + i, &j->timer, true);
 }
 
 // What the front of the one-shot call has done of its run
@@ -2321,12 +2395,12 @@ struct FrontDone {
 // capacity estimated too large costs fixed-point rows only; any other table is built by diff_run_impl once the whole
 // matrix has landed.
 // Split front: the chunks [0, up.split) are processed first and their rows checked against the capacity; the first group's
-// joint then runs while the rest of the matrix is still arriving.  The draws of a are generated while the first chunks'
+// joint then runs while the rest of the matrix is still arriving.  The job's draws are generated while the first chunks'
 // kernels run, into the mapped pinned staging when the front is split.  If the estimate turns out too small the kernels
 // stop at the capacity and *done says what is left: diff_run_impl rebuilds index and table the classic way from the
 // resident counts, and repeats the first joint on the new row ids.
 static int front_chunked(scde_b200_ctx *ctx, scde_b200_diff_job *j, ContractChoice k, CountUpload &up,
-                         const scde_b200_diff_args *a, FrontDone *done) {
+                         FrontDone *done) {
     LpTable &t = j->ws->table;
     const int G = j->G, C = j->C, n_ch = up.chunks();
     cudaStream_t st = ctx->stream;
@@ -2334,7 +2408,7 @@ static int front_chunked(scde_b200_ctx *ctx, scde_b200_diff_job *j, ContractChoi
     const TableRequest req = diff_table(j->models, j->mag.p, j->K, k);
     if (!(plan_table(ctx, req).compact() && C >= 64 * n_ch && ctx->opt.pipeline_front)) {
         TRY(up.wait(0, n_ch));
-        return upload_draws(ctx, j, a);
+        return job_draws(ctx, j);
     }
     const bool split = up.split > 0;
     TRY(index_buffers(ctx, t, G, C));
@@ -2376,7 +2450,7 @@ static int front_chunked(scde_b200_ctx *ctx, scde_b200_diff_job *j, ContractChoi
             SCDE_CUDA(up.drain());
             tr_copy = clk.ms();
         }
-        if (part == 0) TRY(upload_draws(ctx, j, a, split));  // host RNG work while the kernels queued above run
+        if (part == 0) TRY(job_draws(ctx, j, split));  // host RNG work while the kernels queued above run
         const double tr_draws = clk.ms();
         int32_t total = 0, err = 0;
         SCDE_CUDA(cudaMemcpyAsync(&total, t.row_off.p + up.bounds[hi], sizeof(int32_t), cudaMemcpyDeviceToHost, st));
@@ -2396,7 +2470,9 @@ static int front_chunked(scde_b200_ctx *ctx, scde_b200_diff_job *j, ContractChoi
         }
         t.n_rows = total;
         if (split && part == 0) {  // every row of the first group's cells is built and within the capacity
-            TRY(group_joint(ctx, j, k, 0));
+            std::vector<bool> first(j->joints.n_words());
+            first[0] = true;
+            TRY(run_group_joints(ctx, k, t, j->joints, j->dj, first, j->ws->scr, &tm, true));
             done->joint0 = true;
         }
     }
@@ -2405,9 +2481,8 @@ static int front_chunked(scde_b200_ctx *ctx, scde_b200_diff_job *j, ContractChoi
     return SCDE_B200_OK;
 }
 
-// up, a: the one-shot call, whose count matrix is still arriving in chunks and whose draws are still to be made
-static int diff_run_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, ContractChoice k, CountUpload *up = nullptr,
-                         const scde_b200_diff_args *a = nullptr) {
+// up: the one-shot call, whose count matrix is still arriving in chunks and whose draws are still to be made
+static int diff_run_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, ContractChoice k, CountUpload *up = nullptr) {
     if (!j) return SCDE_B200_EINVAL;
     cudaStream_t st = ctx->stream;
     StageTimer &tm = j->timer;
@@ -2416,11 +2491,10 @@ static int diff_run_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, ContractChoi
     SCDE_CUDA(cudaMemsetAsync(j->ws->scr.total.p, 0, 5 * sizeof(unsigned long long), st));
     const int G = j->G, C = j->C, K = j->K;
     const int ld = table_ld(K);
-    SCDE_CUDA(cudaMemsetAsync(j->status.p, 0, 3 * sizeof(int32_t), st));
+    SCDE_CUDA(cudaMemsetAsync(j->dj.status.p, 0, sizeof(int32_t) * j->joints.n_words(), st));
     int t_all = tm.begin(st);
-    const DrawSets sets{j->chunks.n_sets(), j->gene_set.p};
     FrontDone done;
-    if (up) TRY(front_chunked(ctx, j, k, *up, a, &done));
+    if (up) TRY(front_chunked(ctx, j, k, *up, &done));
     j->rows_unchecked = false;
     if (!done.table) {
         // a repeated run of a resident job: the buffers of the last run are exactly large enough, no host round trip (a
@@ -2430,8 +2504,10 @@ static int diff_run_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, ContractChoi
         j->rows_unchecked = known > 0;
         TRY(fill_table(ctx, j->ws->table, diff_table(j->models, j->mag.p, K, k), &tm));
     }
-    for (int i = 0; i < 2; ++i)
-        if (!(i == 0 && done.joint0)) TRY(group_joint(ctx, j, k, i));
+    // the group joints (R/functions.R:372-374), but the first group's when the front has run it
+    std::vector<bool> words(j->joints.n_words(), true);
+    words[0] = !done.joint0;
+    TRY(run_group_joints(ctx, k, j->ws->table, j->joints, j->dj, words, j->ws->scr, &tm, true));
     // batch joints: all cells, composition-sampled draws are global cell ids (R/functions.R:355-357)
     if (j->has_batch) {
         // batch.models differ from models: the table rows are rebuilt from them (same row ids -- the counts have not
@@ -2439,9 +2515,7 @@ static int diff_run_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, ContractChoi
         if (j->bmodels.m.p) TRY(fill_table(ctx, j->ws->table, diff_table(j->bmodels, j->mag.p, K, k), &tm));
         // the two composition-sampled joints walk the same cells and rows with different draws: one launch of the contraction
         // kernel for both, items paired on neighbouring SMs, so the table is pulled from DRAM once for the two
-        const Joint batch[2] = {{j->boot_ptr[2], j->D[2], j->ws->jp[2].p}, {j->boot_ptr[3], j->D[3], j->ws->jp[3].p}};
-        TRY(run_joint(ctx, k, j->ws->table, nullptr, C, batch, 2, j->n_boot, sets, (double)j->n_boot, ld, j->ws->scr,
-                      j->status.p + 2, &tm, true));
+        TRY(run_batch_joints(ctx, k, j->ws->table, j->joints, j->dj, words, j->ws->scr, &tm, true));
     }
     const int e0 = tm.begin(st);
     RatioPasses r = ratio_passes(G, K, ld, j->prior_y.p, j->zi.p, j->zi_adj.p, j->n_zero);
@@ -2492,9 +2566,9 @@ static int diff_download_impl(scde_b200_ctx *ctx, scde_b200_diff_job *j, const s
             }
         }
         j->known_rows = j->ws->table.n_rows;
-        int32_t f[3];
+        std::vector<int32_t> f(j->joints.n_words());
         bool rerun = false;
-        TRY(read_status(j->status.p, f, 3, &rerun));
+        TRY(read_status(j->dj.status.p, f.data(), (int)f.size(), &rerun));
         if (rerun) {  // a multiplicity above 127: repeat the run on the FP64 contraction kernel
             TRY(diff_run_impl(ctx, j, {Contraction::Tiled}));
             SCDE_CUDA(cudaStreamSynchronize(st));
@@ -2543,7 +2617,7 @@ int scde_b200_diff_upload(scde_b200_ctx *ctx, const scde_b200_diff_args *a, int3
     *out = nullptr;
     JobPtr j;
     TRY(diff_upload_impl(ctx, a, want_posteriors, j));
-    TRY(upload_draws(ctx, j.get(), a));
+    TRY(job_draws(ctx, j.get()));
     // the counts shard, rows [gene_begin, gene_end) of every column, in one copy that has landed when the call returns
     const WallClock clk;
     SCDE_CUDA(j->ws->counts.ensure((size_t)j->G * j->C));
@@ -2590,7 +2664,7 @@ static int expression_difference_single(scde_b200_ctx *ctx, const scde_b200_diff
     CountUpload up(ctx);
     TRY(up.start(*job, args->counts + args->gene_begin, args->n_genes));
     const double t_up = clk.ms();
-    int r = diff_run_impl(ctx, job.get(), k, &up, args);
+    int r = diff_run_impl(ctx, job.get(), k, &up);
     const double t_run = clk.ms();
     if (r == SCDE_B200_OK) r = diff_download_impl(ctx, job.get(), out, stats, pl, k);
     const double t_down = clk.ms();
@@ -2650,16 +2724,9 @@ struct ContrastPlan {
     int C = 0, K = 0, N = 0;          // cells, grid points, genes of the dataset
     int n_contrasts = 0, n_boot = 0;
     bool has_batch = false, want_post = false;
-    std::vector<int> slot_group;      // bank slot -> group id (only groups some contrast names)
-    std::vector<int32_t> cells;       // the slots' cells back to back
-    std::vector<int64_t> cell_off;    // slot -> offset into cells (n_slots + 1)
-    int seed = 1, draw_chunks = 0;    // the draw sets: DrawChunks over the dataset's genes
-    int n_sets = 1;                   // draw sets over all genes (a shard uses those of the chunks it meets)
-    std::vector<int32_t> draws;       // group draws per distinct group size: n_sets blocks of n_boot x size
-    std::vector<int64_t> draw_off;    // slot -> offset into draws
-    std::vector<int> bslot_D;         // batch slot (distinct composition) -> draws per boot
-    std::vector<int32_t> bdraws;      // batch draws (global cell ids) per batch slot: n_sets blocks of n_boot x D
-    std::vector<int64_t> bdraw_off;
+    std::vector<int> slot_group;      // bank slot (group joint) -> group id (only groups some contrast names)
+    JointPlan joints;                 // a group joint per slot, a batch joint per batch slot (distinct composition)
+    std::unique_ptr<int32_t[]> draws; // every draw set of the joints (generate_draws; a shard uploads those it meets)
     std::vector<int> pair_slot, pair_bslot;  // 2 per contrast
     std::vector<int32_t> zi, zi_adj;  // n_zero entries each (1 or N)
     int n_zero = 1;
@@ -2681,7 +2748,8 @@ struct DatasetShard {
     int rows_from = 0;
     bool rows_i8 = false;
     DBuf<double> bank, bbank;                 // joint posteriors, [slot][G][ld]
-    DBuf<int32_t> cells, draws, bdraws, zi, zi_adj, jflags, gene_set;
+    JointDevice joints;
+    DBuf<int32_t> zi, zi_adj;
     DBuf<int32_t> idx, bidx, aidx;            // [contrast][3][G]
     DBuf<double> z, bz, az;                   // [contrast][G]
     DBuf<RatioContrast> rtab;                 // [pass][contrast] device tables of the batched ratio launches
@@ -2774,50 +2842,16 @@ int shard_contrasts(DatasetShard &sh, const ContrastPlan &p, const scde_b200_con
     const ContractChoice k = contraction_choice(ctx);
     const int G = sh.G, K = sh.K, nc = p.n_contrasts;
     const int ld = t.ld, nout = 2 * K - 1, ldo = round_up(nout, 8), nadj = 2 * nout - 1, lda = round_up(nadj, 8);
-    const int n_slots = (int)p.slot_group.size(), n_bslots = (int)p.bslot_D.size();
+    const JointPlan &jp = p.joints;
+    const int n_slots = jp.n_groups(), n_bslots = (int)jp.batch_block.size();
     SCDE_CUDA(ws->scr.total.ensure(5));
     SCDE_CUDA(cudaMemsetAsync(ws->scr.total.p, 0, 5 * sizeof(unsigned long long), st));
     const int t_all = tm.begin(st);
     TRY(ensure_rows(sh, 0, k, &tm));
-    TRY(upload(sh.cells, p.cells.data(), p.cells.size(), st));
-    // this shard's draw sets: those of the chunks it meets.  Only they are uploaded, packed per group size (and per batch
-    // composition); sh_draw_off / sh_bdraw_off map a plan offset (the block of all sets) to the packed block on the device.
-    const DrawChunks dc = draw_chunks_of(p.N, p.draw_chunks, p.seed, sh.g0, sh.g0 + G);
-    std::map<int64_t, int64_t> sh_draw_off;
-    std::vector<int64_t> sh_bdraw_off(p.bdraw_off.size());
-    {
-        auto pack = [&](DBuf<int32_t> &buf, const std::vector<int32_t> &all, const std::vector<std::pair<int64_t, int64_t>> &blocks,
-                        std::vector<int64_t> &local) -> int {  // blocks: (plan offset, draws per set)
-            int64_t total = 0;
-            for (const auto &b : blocks) total += (int64_t)dc.n_sets() * b.second;
-            SCDE_CUDA(buf.ensure((size_t)(total > 0 ? total : 1)));
-            int64_t off = 0;
-            local.clear();
-            for (const auto &b : blocks) {
-                local.push_back(off);
-                const int64_t n = (int64_t)dc.n_sets() * b.second;
-                if (n > 0)
-                    SCDE_CUDA(cudaMemcpyAsync(buf.p + off, all.data() + b.first + (int64_t)dc.first * b.second,
-                                              sizeof(int32_t) * n, cudaMemcpyHostToDevice, st));
-                off += n;
-            }
-            return SCDE_B200_OK;
-        };
-        std::vector<std::pair<int64_t, int64_t>> blocks;
-        for (int s = 0; s < n_slots; ++s)
-            if (!sh_draw_off.count(p.draw_off[s])) {
-                sh_draw_off[p.draw_off[s]] = -1;
-                blocks.emplace_back(p.draw_off[s], (int64_t)p.n_boot * (p.cell_off[s + 1] - p.cell_off[s]));
-            }
-        std::vector<int64_t> local;
-        TRY(pack(sh.draws, p.draws, blocks, local));
-        for (size_t i = 0; i < blocks.size(); ++i) sh_draw_off[blocks[i].first] = local[i];
-        if (p.has_batch) {
-            blocks.clear();
-            for (int b = 0; b < n_bslots; ++b) blocks.emplace_back(p.bdraw_off[b], (int64_t)p.n_boot * p.bslot_D[b]);
-            TRY(pack(sh.bdraws, p.bdraws, blocks, sh_bdraw_off));
-        }
-    }
+    // this shard's draw sets: those of the chunks it meets
+    const DrawChunks dc = jp.sets_of(sh.g0, sh.g0 + G);
+    TRY(place_joints(ctx, jp, dc, sh.joints));
+    TRY(upload_draws(ctx, jp, dc, p.draws.get(), sh.joints));
     {
         const std::vector<int32_t> zi = zero_slice(p.zi.data(), p.n_zero, sh.g0, G);
         TRY(upload(sh.zi, zi.data(), zi.size(), st));
@@ -2832,55 +2866,34 @@ int shard_contrasts(DatasetShard &sh, const ContrastPlan &p, const scde_b200_con
     const size_t slot_sz = (size_t)G * ld;
     SCDE_CUDA(sh.bank.ensure((size_t)n_slots * slot_sz));
     if (p.has_batch) SCDE_CUDA(sh.bbank.ensure((size_t)n_bslots * slot_sz));
-    // tcgen05 status words, one per group joint and per pair of batch joints: a flagged joint is recomputed alone below
-    const int n_words = n_slots + (n_bslots + 1) / 2;
-    SCDE_CUDA(sh.jflags.ensure((size_t)n_words));
-    SCDE_CUDA(cudaMemsetAsync(sh.jflags.p, 0, sizeof(int32_t) * n_words, st));
-    if (dc.n_sets() > 1) {
-        TRY(upload(sh.gene_set, dc.gene_set.data(), dc.gene_set.size(), st));
-        SCDE_CUDA(cudaStreamSynchronize(st));
-    }
-    const DrawSets sets{dc.n_sets(), dc.n_sets() > 1 ? sh.gene_set.p : nullptr};
-    auto group_draws = [&](int s) { return sh.draws.p + sh_draw_off.at(p.draw_off[s]); };
-    auto batch_draws = [&](int b) { return sh.bdraws.p + sh_bdraw_off[b]; };
-    auto group_joint = [&](int s, ContractChoice kk, bool count) {
-        const int n = (int)(p.cell_off[s + 1] - p.cell_off[s]);
-        const Joint jt{group_draws(s), n, sh.bank.p + s * slot_sz};
-        return run_joint(ctx, kk, t, sh.cells.p + p.cell_off[s], n, &jt, 1, p.n_boot, sets, (double)p.n_boot, ld, ws->scr,
-                         sh.jflags.p + s, &tm, count);
-    };
-    // batch joints b .. b + n - 1 (n <= 2); a pair of joints shares status word n_slots + b / 2
-    auto batch_joints = [&](int b, int n, ContractChoice kk, bool count) {
-        auto joint = [&](int i) { return Joint{batch_draws(i), p.bslot_D[i], sh.bbank.p + i * slot_sz}; };
-        const Joint js[2] = {joint(b), joint(b + n - 1)};
-        return run_joint(ctx, kk, t, nullptr, sh.C, js, n, p.n_boot, sets, (double)p.n_boot, ld, ws->scr,
-                         sh.jflags.p + n_slots + b / 2, &tm, count);
-    };
-    for (int s = 0; s < n_slots; ++s) TRY(group_joint(s, k, true));
+    sh.joints.jp.clear();  // joint -> its bank slot
+    for (int s = 0; s < n_slots; ++s) sh.joints.jp.push_back(sh.bank.p + s * slot_sz);
+    for (int b = 0; b < n_bslots; ++b) sh.joints.jp.push_back(sh.bbank.p + b * slot_sz);
+    // a status word per group joint and per pair of batch joints: a flagged joint is recomputed alone below
+    const int n_words = jp.n_words();
+    SCDE_CUDA(cudaMemsetAsync(sh.joints.status.p, 0, sizeof(int32_t) * n_words, st));
+    const std::vector<bool> all(n_words, true);
+    TRY(run_group_joints(ctx, k, t, jp, sh.joints, all, ws->scr, &tm, true));
     if (p.has_batch) {
         if (p.batch_models) TRY(ensure_rows(sh, 1, k, &tm));
         // distinct compositions in pairs: one launch of the tcgen05 kernel for two joints over the same cells and rows
-        for (int b = 0; b < n_bslots; b += 2) TRY(batch_joints(b, n_bslots - b < 2 ? 1 : 2, k, true));
+        TRY(run_batch_joints(ctx, k, t, jp, sh.joints, all, ws->scr, &tm, true));
     }
     SCDE_CUDA(cudaStreamSynchronize(st));
     std::vector<int32_t> flags(n_words);
     bool any = false;
-    TRY(read_status(sh.jflags.p, flags.data(), n_words, &any));
+    TRY(read_status(sh.joints.status.p, flags.data(), n_words, &any));
     if (any) {  // only the flagged joints are repeated, on the FP64 kernel (FP64 table rows)
-        bool rows = false;
-        for (int s = 0; s < n_slots; ++s)
-            if (flags[s] & (1 | 4)) {
-                if (!rows) TRY(ensure_rows(sh, 0, {Contraction::Tiled}, &tm));
-                rows = true;
-                TRY(group_joint(s, {Contraction::Tiled}, false));
-            }
-        rows = false;
-        for (int b = 0; b < n_bslots; ++b)
-            if (flags[n_slots + b / 2] & (1 | 4)) {
-                if (!rows) TRY(ensure_rows(sh, p.batch_models ? 1 : 0, {Contraction::Tiled}, &tm));
-                rows = true;
-                TRY(batch_joints(b, 1, {Contraction::Tiled}, false));
-            }
+        std::vector<bool> redo(n_words);
+        for (int w = 0; w < n_words; ++w) redo[w] = (flags[w] & (1 | 4)) != 0;
+        if (std::count(redo.begin(), redo.begin() + n_slots, true)) {
+            TRY(ensure_rows(sh, 0, {Contraction::Tiled}, &tm));
+            TRY(run_group_joints(ctx, {Contraction::Tiled}, t, jp, sh.joints, redo, ws->scr, &tm, false));
+        }
+        if (std::count(redo.begin() + n_slots, redo.end(), true)) {
+            TRY(ensure_rows(sh, p.batch_models ? 1 : 0, {Contraction::Tiled}, &tm));
+            TRY(run_batch_joints(ctx, {Contraction::Tiled}, t, jp, sh.joints, redo, ws->scr, &tm, false));
+        }
     }
     // ratio and summary: every contrast in one launch per pass; the 2K-1 posteriors that feed the adjusted pass (or that
     // the caller wants) exist only for a block of contrasts at a time, sized to the free device memory
@@ -2998,11 +3011,12 @@ int plan_contrasts(const scde_b200_dataset *ds, const scde_b200_contrast_args *a
         return bad("contrasts: zero_index (and zero_index_adjusted with batch) are required");
     TRY(validate_index(a->zero_index, (size_t)a->n_zero, 1, 2 * K, "zero_index"));
     p.zi.assign(a->zero_index, a->zero_index + a->n_zero);
-    BatchPools bp;  // the draw pools of the batch joints below
+    JointPlan &jp = p.joints;
+    jp = JointPlan(C, a->n_boot, N, a->draw_chunks, a->seed, 0, N);
     if (p.has_batch) {
         TRY(validate_index(a->zero_index_adjusted, (size_t)a->n_zero, 1, 4 * K - 2, "zero_index_adjusted"));
         p.zi_adj.assign(a->zero_index_adjusted, a->zero_index_adjusted + a->n_zero);
-        TRY(batch_pools(a->batch, C, a->n_batch_levels, bp));
+        TRY(batch_pools(a->batch, C, a->n_batch_levels, jp.pools));
     }
     p.C = C;
     p.K = K;
@@ -3010,10 +3024,6 @@ int plan_contrasts(const scde_b200_dataset *ds, const scde_b200_contrast_args *a
     p.n_zero = a->n_zero;
     p.n_contrasts = a->n_contrasts;
     p.n_boot = a->n_boot;
-    p.seed = a->seed;
-    p.draw_chunks = a->draw_chunks;
-    const std::vector<int32_t> seeds = chunk_seeds(N, a->draw_chunks, a->seed);
-    p.n_sets = (int)seeds.size();
     p.want_post = o->difference_posterior || o->adjusted_difference_posterior;
     std::vector<int> slot_of(a->n_groups, -1);
     p.pair_slot.resize(2 * (size_t)a->n_contrasts);
@@ -3038,62 +3048,47 @@ int plan_contrasts(const scde_b200_dataset *ds, const scde_b200_contrast_args *a
             p.pair_slot[2 * c + s] = slot_of[g];
         }
     }
-    // group joints: cells of every slot, draws once per distinct group size (local indices, src/jpmatLogBoot.cpp:221,254-257)
-    // and draw set; the draws are generated below, on parallel host threads, one (size or composition, set) each
-    const int S = p.n_sets;
-    std::vector<std::pair<int64_t, int>> group_tasks;  // (offset of the set's block, size)
-    std::map<int, int64_t> draws_of_size;
-    p.cell_off.assign(1, 0);
+    // group joints: one per slot, a draw block per distinct group size (local indices)
+    std::map<int, int> block_of_size;
     for (int g : p.slot_group) {
         const int32_t b = a->group_offsets[g], e = a->group_offsets[g + 1];
-        p.cells.insert(p.cells.end(), a->group_cells + b, a->group_cells + e);
-        p.cell_off.push_back((int64_t)p.cells.size());
-        const int n = e - b;
-        auto it = draws_of_size.find(n);
-        if (it == draws_of_size.end()) {
-            it = draws_of_size.emplace(n, (int64_t)p.draws.size()).first;
-            for (int s = 0; s < S; ++s) group_tasks.emplace_back(it->second + (int64_t)s * a->n_boot * n, n);
-            p.draws.resize(p.draws.size() + (size_t)S * a->n_boot * n);
+        jp.cells.insert(jp.cells.end(), a->group_cells + b, a->group_cells + e);
+        jp.cell_off.push_back((int64_t)jp.cells.size());
+        auto it = block_of_size.find(e - b);
+        if (it == block_of_size.end()) {
+            it = block_of_size.emplace(e - b, (int)jp.blocks.size()).first;
+            jp.blocks.push_back(DrawBlock{e - b});
         }
-        p.draw_off.push_back(it->second);
+        jp.group_block.push_back(it->second);
     }
-    TRY(parallel_for((int)group_tasks.size(), [&](int i) -> int {
-        const auto &tk = group_tasks[i];
-        return scde_b200_boot_indices(seeds[(size_t)i % S], tk.second, a->n_boot, p.draws.data() + tk.first);
-    }));
-    if (!p.has_batch) return SCDE_B200_OK;
-    // batch joints: one per distinct composition table(batch[group]) (R/functions.R:355-357)
-    const int L = a->n_batch_levels;
-    std::map<std::vector<int32_t>, int> bslot_of;
-    std::vector<std::vector<int32_t>> bcomp;  // composition of every batch slot
-    std::vector<int> bslot_of_slot(p.slot_group.size());
-    for (size_t s = 0; s < p.slot_group.size(); ++s) {
-        std::vector<int32_t> comp;
-        const int D = batch_composition(a->batch, L, p.cells.data() + p.cell_off[s], (size_t)(p.cell_off[s + 1] - p.cell_off[s]),
-                                        comp);
-        auto it = bslot_of.find(comp);
-        if (it == bslot_of.end()) {
-            it = bslot_of.emplace(comp, (int)p.bslot_D.size()).first;
-            p.bslot_D.push_back(D);
-            p.bdraw_off.push_back((int64_t)p.bdraws.size());
-            p.bdraws.resize(p.bdraws.size() + (size_t)S * a->n_boot * D);
-            bcomp.push_back(comp);
+    if (p.has_batch) {
+        // batch joints: one per distinct composition table(batch[group]) (R/functions.R:355-357), each with its block
+        std::map<std::vector<int32_t>, int> bslot_of;
+        std::vector<int> bslot_of_slot(p.slot_group.size());
+        for (size_t s = 0; s < p.slot_group.size(); ++s) {
+            DrawBlock k;
+            k.batch = true;
+            k.D = batch_composition(a->batch, a->n_batch_levels, jp.cells.data() + jp.cell_off[s],
+                                    (size_t)(jp.cell_off[s + 1] - jp.cell_off[s]), k.comp);
+            auto it = bslot_of.find(k.comp);
+            if (it == bslot_of.end()) {
+                it = bslot_of.emplace(k.comp, (int)jp.batch_block.size()).first;
+                jp.batch_block.push_back((int)jp.blocks.size());
+                jp.blocks.push_back(std::move(k));
+            }
+            bslot_of_slot[s] = it->second;
         }
-        bslot_of_slot[s] = it->second;
+        p.pair_bslot.resize(p.pair_slot.size());
+        for (size_t i = 0; i < p.pair_slot.size(); ++i) p.pair_bslot[i] = bslot_of_slot[p.pair_slot[i]];
+        if (a->batch_models) {
+            p.batch_models = a->batch_models;
+            p.batch_local_theta = a->batch_local_theta;
+            p.batch_sqlogit = a->batch_square_logit_conc;
+        }
     }
-    TRY(parallel_for((int)bcomp.size() * S, [&](int i) -> int {
-        const int b = i / S, set = i % S;
-        return scde_b200_batch_boot_indices(seeds[set], L, bp.off.data(), bp.pool.data(), bcomp[b].data(), a->n_boot,
-                                            p.bdraws.data() + p.bdraw_off[b] + (int64_t)set * a->n_boot * p.bslot_D[b]);
-    }));
-    p.pair_bslot.resize(p.pair_slot.size());
-    for (size_t i = 0; i < p.pair_slot.size(); ++i) p.pair_bslot[i] = bslot_of_slot[p.pair_slot[i]];
-    if (a->batch_models) {
-        p.batch_models = a->batch_models;
-        p.batch_local_theta = a->batch_local_theta;
-        p.batch_sqlogit = a->batch_square_logit_conc;
-    }
-    return SCDE_B200_OK;
+    // every draw set of every block once per call, on parallel host threads
+    p.draws.reset(new int32_t[jp.block_off((int)jp.blocks.size(), jp.sets.n_sets())]);
+    return generate_draws(jp, p.draws.get(), false);
 }
 
 }  // namespace
